@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]
                     [--workload target|config1|config2|config3|config4|config5]
-                    [--impl b200|reference] [--scaling strong|weak]
+                    [--impl b200|reference] [--scaling strong|weak] [--dump-outputs DIR]
 
 Default workload: the north-star TARGET (2 000 samples x 20 000 features, 25 % left-censored,
 1 999 000 pairs), which fits one GPU.  N > 1 (torchrun, one rank per GPU) defaults to STRONG scaling
@@ -19,6 +19,10 @@ region) through the public call -- the one-shot C ABI `icikt_all_pairs` at N = 1
 torchrun; `e2e_pageable` repeats it from a plain NumPy array into freshly allocated outputs, which is
 what an R caller hands over.  After the timed region a seeded sample of pairs is checked against the
 CPU oracle (`parity_sample`).
+
+--dump-outputs DIR writes what the timed plan returned for its last step as DIR/<name>.npy (see
+dump_outputs).  The inputs are seeded, so two builds run with the same arguments can be compared
+array for array.
 
 --impl reference times the reference's CPU path.  R and Rcpp are not installed in this image, so
 the true Rcpp+furrr path cannot run; the arm times the line-faithful C++ restatement (oracle/,
@@ -39,9 +43,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "column-pairs/sec"
 P_TOL = 1e-12  # p-value: |dp| <= P_TOL * max(1, z^2) * p  (relative error of a normal tail ~ z^2 eps)
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much
+DUMP_SEED = 7001
 
 
 def w_smem(n):
@@ -216,6 +223,28 @@ def parity_sample(x, persp, got, lo, hi, n_sample, device):
     return out
 
 
+def dump_outputs(out_dir, res, P):
+    """Writes the per-pair results `res` (all P pairs in pair order, as Plan.download returns them) to
+    out_dir/<name>.npy: raw, pvalue, taumax, completeness (float64), status (float32), max_taumax
+    (float64, one element) and pair_index (float64), the positions in the pair order of the pairs
+    written.  All pairs when they fit in DUMP_BYTES, otherwise a seeded random sample that depends
+    only on P, so that runs of the same workload write the same pairs."""
+    per_pair = 4 * 8 + 4 + 8
+    m = min(P, (DUMP_BYTES - 4096) // per_pair)  # 4096: the .npy headers
+    if m == P:
+        sel = np.arange(P)
+    else:
+        sel = np.sort(np.random.default_rng(DUMP_SEED).choice(P, size=m, replace=False))
+    arrays = {k: np.ascontiguousarray(res[k][sel], dtype=np.float64)
+              for k in ("raw", "pvalue", "taumax", "completeness")}
+    arrays["status"] = res["status"][sel].astype(np.float32)
+    arrays["max_taumax"] = np.array([res["max_taumax"]], dtype=np.float64)
+    arrays["pair_index"] = sel.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -234,7 +263,13 @@ def main():
     ap.add_argument("--quick", action="store_true", help="skip the e2e, parity and CPU legs (tuning sweeps)")
     ap.add_argument("--parity-pairs", type=int, default=320)
     ap.add_argument("--replicate-k1", action="store_true", help="N > 1: every rank preprocesses all columns")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed plan's results of the last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a sample of pairs, not the whole result")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -334,7 +369,15 @@ def main():
     dev_ms = max_over_ranks(dev_ms)
     clocks = sampler.stop()
     value = P_total * args.steps / (dev_ms * 1e-3)
-    got = plan.download() if not args.quick else None  # the timed plan's results of this rank's slice
+    # the timed plan's results of this rank's slice
+    got = plan.download() if not args.quick or args.dump_outputs else None
+    if args.dump_outputs:
+        parts = [got]
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, got)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, sharding.gather_results(parts, P_total), P_total)
 
     # ---- e2e: host buffers in, host results out, every step uploads and downloads ----
     e2e_kw = dict(perspective=persp, device=local_rank, kernel=kernel, pair_lo=lo, pair_hi=hi)

@@ -56,7 +56,8 @@ def make(name, n=None, C=None, seed=None):
     seed = SEEDS[name] if seed is None else seed
     if kind == "yeast":
         # BASELINE config 1: the reference's bundled yeast RNA-seq counts (6 887 x 96), zeros -> missing
-        # as ici_kendalltau's default global_na does; fixture made by tests/golden/make_golden.py
+        # as ici_kendalltau's default global_na does; fixture made by tests/golden/make_golden.py (stored as
+        # per-column ranks, which give the pair results of the original values)
         import os
         here = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
         x = np.array(np.load(os.path.join(here, "tests", "golden", "yeast_missing.npz"))["data"], dtype=np.float64)

@@ -1,13 +1,16 @@
 """tests/golden/make_golden.py -- regenerates the committed fixtures in tests/golden/.
 
-Run in the BUILD container (needs /root/reference; the GPU box does not have it):
+Needs a checkout of the reference R package (no R itself):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 Outputs
   yeast_missing.npz      data/yeast_missing.rda of the reference converted to NumPy
-                         (6887 features x 96 samples, fp64, column names), read with
-                         the small XDR reader below -- no R needed.
+                         (6887 features x 96 samples, column names), read with the small
+                         XDR reader below.  Stored as per-column dense ranks (uint16; 0 where
+                         the value is 0, i.e. missing): every pair statistic depends only on
+                         the order and ties within each column and on which entries are
+                         missing, so results are those of the original values, in under 1 MB.
   yeast_oracle.npz       oracle (oracle/icikt_oracle.cpp) results for all 4560 column
                          pairs of yeast_missing, global and local perspective:
                          tau/pvalue/tau_max/completeness/status + int64 counts.
@@ -31,7 +34,6 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
 
 
 class _XDR:
@@ -135,8 +137,8 @@ def read_rda(path):
     return x.item()
 
 
-def load_yeast():
-    top = read_rda(os.path.join(REF, "data", "yeast_missing.rda"))
+def load_yeast(ref):
+    top = read_rda(os.path.join(ref, "data", "yeast_missing.rda"))
     (tag, (kind, vals, attr)), = top
     assert tag == "yeast_missing" and kind == "real", (tag, kind)
     dim = attr["dim"][1]
@@ -146,13 +148,24 @@ def load_yeast():
     return data, colnames
 
 
-def main():
+def column_ranks(data):
+    """Dense ranks of the positive values of every column, from 1; zeros stay 0."""
+    assert (data >= 0).all()
+    out = np.zeros(data.shape, dtype=np.uint16)
+    for j in range(data.shape[1]):
+        pos = data[:, j] > 0
+        _, inv = np.unique(data[pos, j], return_inverse=True)
+        assert inv.size == 0 or inv.max() + 1 < 2 ** 16
+        out[pos, j] = inv + 1
+    return out
+
+
+def main(ref):
     from oracle import oracle as O
 
-    data, colnames = load_yeast()
+    data, colnames = load_yeast(ref)
     print("yeast_missing", data.shape, "zeros:", int((data == 0).sum()))
-    np.savez_compressed(os.path.join(HERE, "yeast_missing.npz"), data=data.astype(np.float64),
-                        colnames=colnames)
+    np.savez_compressed(os.path.join(HERE, "yeast_missing.npz"), data=column_ranks(data), colnames=colnames)
 
     excl = O.setup_missing_matrix(data)
     ex = data.copy()
@@ -201,4 +214,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

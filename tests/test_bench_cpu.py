@@ -28,6 +28,45 @@ def test_reference_arm_line_and_workload_label():
     assert 'add_argument("--workload", default="target"' in src and 'add_argument("--scaling", default="strong"' in src
 
 
+def test_dump_outputs_full_and_sampled(tmp_path, monkeypatch):
+    """--dump-outputs: float32/float64 .npy files within the byte budget; a larger result set is written as
+    the same seeded sample of pairs on every run, with the pairs' positions in pair_index."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    P = 5000
+    rng = np.random.default_rng(1)
+    res = {k: rng.normal(size=P) for k in ("raw", "pvalue", "taumax", "completeness")}
+    res["status"] = rng.integers(0, 5, size=P).astype(np.int32)
+    res["max_taumax"] = 0.75
+
+    def load(d):
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+
+    bench.dump_outputs(str(tmp_path / "full"), res, P)
+    full = load(tmp_path / "full")
+    assert sorted(full) == ["completeness", "max_taumax", "pair_index", "pvalue", "raw", "status", "taumax"]
+    assert all(v.dtype in (np.float32, np.float64) for v in full.values())
+    assert np.array_equal(full["pair_index"], np.arange(P)) and full["max_taumax"].tolist() == [0.75]
+    assert np.array_equal(full["raw"], res["raw"]) and np.array_equal(full["status"], res["status"])
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 44 * 1000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), res, P)
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= bench.DUMP_BYTES
+    sel = a["pair_index"].astype(np.int64)
+    assert sel.size == 1000 and np.all(np.diff(sel) > 0)
+    for k in ("raw", "pvalue", "taumax", "completeness", "status"):
+        assert np.array_equal(a[k], res[k][sel]) and np.array_equal(a[k], b[k]), k
+
+
+def test_steps_must_be_positive():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="3", WORLD_SIZE="8", LOCAL_RANK="3")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "8"],

@@ -99,7 +99,7 @@ def test_yeast_missing_matches_golden(golden_dir, persp):
     """BASELINE config 1: ici_kendalltau(yeast_missing), all 4560 pairs, vs committed oracle output."""
     d = np.load(os.path.join(golden_dir, "yeast_missing.npz"))
     o = np.load(os.path.join(golden_dir, "yeast_oracle.npz"))
-    got = ik.run_pairs(d["data"], (np.nan, np.inf, 0.0), perspective=persp, want_counts=True)
+    got = ik.run_pairs(d["data"].astype(np.float64), (np.nan, np.inf, 0.0), perspective=persp, want_counts=True)
     ref = {k: o[f"{persp}_{k}"] for k in ("raw", "pvalue", "taumax", "completeness", "status", "counts")}
     assert_parity(got, ref, f"yeast {persp}")
     # SURVEY.md 8c: Snf2.01 x Snf2.02
@@ -111,8 +111,9 @@ def test_yeast_missing_matches_golden(golden_dir, persp):
 def test_yeast_ici_kendalltau_api(golden_dir):
     d = np.load(os.path.join(golden_dir, "yeast_missing.npz"))
     names = [str(s) for s in d["colnames"]]
-    got = ik.ici_kendalltau(d["data"], colnames=names)
-    ref = O.ici_kendalltau(d["data"], ncore=os.cpu_count() or 1)
+    data = d["data"].astype(np.float64)
+    got = ik.ici_kendalltau(data, colnames=names)
+    ref = O.ici_kendalltau(data, ncore=os.cpu_count() or 1)
     for k in ("cor", "raw", "pvalue", "taumax", "completeness"):
         np.testing.assert_allclose(got[k], ref[k], rtol=1e-12, atol=0, err_msg=k)
     assert np.array_equal(got["keep"], ref["keep"])

@@ -219,7 +219,7 @@ def test_local_equals_global_counts_formula():
 def test_yeast_fixture_is_current(golden_dir):
     d = np.load(os.path.join(golden_dir, "yeast_missing.npz"))
     o = np.load(os.path.join(golden_dir, "yeast_oracle.npz"))
-    data = d["data"]
+    data = d["data"].astype(np.float64)
     assert data.shape == (6887, 96)
     ex = data.copy()
     ex[O.setup_missing_matrix(data)] = np.nan
