@@ -35,7 +35,6 @@ def _stale(target: str, deps) -> bool:
 
 def build(force: bool = False, verbose: bool = False) -> str:
     nvcc = _nvcc()
-    extra = os.environ.get("ICIKT_NVCC_EXTRA", "").split()  # tuning experiments only (-D..., -Xptxas ...)
     objdir = os.path.join(CSRC, "build")
     os.makedirs(objdir, exist_ok=True)
     hdrs = [os.path.join(CSRC, h) for h in HEADERS]
@@ -45,7 +44,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
         o = os.path.join(objdir, src.replace(".cu", ".o"))
         objs.append(o)
         if force or _stale(o, [s] + hdrs):
-            cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", s, "-o", o]
+            cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", s, "-o", o]
             procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)))
     for cmd, pr in procs:
         out, _ = pr.communicate()

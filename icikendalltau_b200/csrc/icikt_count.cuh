@@ -7,22 +7,10 @@
 
 #include <cstdint>
 
-// unroll factors of pass A's two sweeps over a thread's 8-key runs (tuning knobs; 1 = one run per iteration)
-#ifndef ICIKT_COUNT_UNROLL
-#define ICIKT_COUNT_UNROLL 1
-#endif
-#ifndef ICIKT_HI_KEY_MASKS
-#define ICIKT_HI_KEY_MASKS 1
-#endif
-#ifndef ICIKT_SCATTER_UNROLL
-#define ICIKT_SCATTER_UNROLL 1
-#endif
-
 namespace icikt {
 namespace {
 
 constexpr unsigned FULL = 0xffffffffu;
-constexpr int kCountUnroll = ICIKT_COUNT_UNROLL, kScatterUnroll = ICIKT_SCATTER_UNROLL;
 
 __device__ __forceinline__ uint32_t lanemask_lt() {
   uint32_t m;
@@ -325,7 +313,7 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     const typename M::ptr ra = M::add(a, (int32_t)my_off);
     uint32_t cl = 0, cb = 0, wm = 0, m4 = 0;
     uint32_t chj[4] = {0u, 0u, 0u, 0u};
-#pragma unroll kCountUnroll
+#pragma unroll 1
     for (int c = 0; c < (idle ? 0 : kk); ++c) {
       uint32_t w[4];
       M::ld128(M::add(ra, c << 4), w[0], w[1], w[2], w[3]);
@@ -374,19 +362,14 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     if (idle) {
       // nothing to move, nothing to count
     } else if (s > 0) {
-#pragma unroll kScatterUnroll
+#pragma unroll 1
       for (int c = 0; c < kk; ++c) {
         uint32_t w[4];
         M::ld128(M::add(ra, c << 4), w[0], w[1], w[2], w[3]);
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           M::step4(Q01, Q23, acc2, w[j], bLl, bHl, w[j], b, pc);
-#if ICIKT_HI_KEY_MASKS
           M::step4(Q01, Q23, acc2, w[j], bLh, bHh, M::hi16(w[j], pc.c64k), b, pc);
-#else
-          const uint32_t kh = M::hi16(w[j], pc.c64k);  // the odd key, tested with the even key's masks
-          M::step4(Q01, Q23, acc2, kh, bLl, bHl, kh, b, pc);
-#endif
         }
       }
     } else {  // the sorted sequence itself is not needed: the last level only counts

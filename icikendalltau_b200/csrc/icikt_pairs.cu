@@ -34,12 +34,13 @@
 //   clz) survives only as tier 2, for columns with very many large groups x distinct values.
 //   When y is (nearly) tie-free the first group's histogram shrinks to ONE BIT per rank, set from the
 //   membership masks (popc(first_x & missing_y) rows are only counted), see group_hist.
-//   Long vectors (the in-place variant, IP != 0) order the work differently: staged_gather fills
-//   every position through a rank table that passes through the idle counter area in TMA parts,
-//   small_groups_inplace compares on the sequence itself, large_groups_sorted2 sorts the first
-//   group together with the large ones.  Those routines exist only in the long-vector
-//   instantiations: the same edits in the short-vector kernel cost it 2-3 % through register
-//   allocation (profiles/r02_build_variants_ab.txt).
+//   Long vectors (global scratch G, or in place IP != 0: y's rank table is not staged) order the
+//   work differently: small_groups_inplace compares on the sequence itself after the gather, and
+//   large_groups_sorted2 sorts the large groups; in place, staged_gather fills every position
+//   through a rank table that passes through the idle counter area in TMA parts, and
+//   large_groups_sorted2 sorts the first group together with the large ones.  Those routines exist
+//   only in the long-vector instantiations: the same edits in the short-vector kernel cost it 2-3 %
+//   through register allocation (profiles/r02_build_variants_ab.txt).
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -262,16 +263,6 @@ __device__ __forceinline__ void count_pass_inplace(const uint32_t a, const int n
 }
 
 // Per-thread sums of the complete-observations mode for one side of a pair (see group_hist).
-// ICIKT_BITMAP_EMIT: group_hist's one-bit-per-rank fast path
-#ifndef ICIKT_BITMAP_EMIT
-#define ICIKT_BITMAP_EMIT 1
-#endif
-constexpr bool kBitmapEmit = ICIKT_BITMAP_EMIT != 0;
-// ICIKT_BITMAP_BY_MASK: the fast path walks the group's membership mask instead of its row list
-#ifndef ICIKT_BITMAP_BY_MASK
-#define ICIKT_BITMAP_BY_MASK 1
-#endif
-constexpr bool kBitmapByMask = ICIKT_BITMAP_BY_MASK != 0;
 struct PwSide {
   unsigned long long S = 0;   // sum over the group's rows of (present rows of the other column below it)
   unsigned long long T = 0;   // ties of the group's present rows in the other column, sum C(count, 2)
@@ -319,7 +310,7 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
     hw = 16;
     hist = M::from_shared(mini);
   }
-  if (kBitmapEmit && EMIT && !PW && try_bits && ((K + 31) >> 5) <= hw) {
+  if (EMIT && !PW && try_bits && ((K + 31) >> 5) <= hw) {
     // Fast path for the usual case -- apart from the other column's lowest rank (rows missing in both
     // columns, counted by ballot) no two rows of the group share a rank: ONE BIT per rank instead of a
     // counter.  K / 32 words to clear, scan and walk instead of K / 2 (x's 5 000 missing rows over y's
@@ -330,7 +321,11 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
     for (int w = tid; w < bw; w += T) M::st32(M::add(bits, w << 2), 0u);
     if (tid == 0) mini[17] = 0u;
     __syncthreads();
-    if (kBitmapByMask && grp_bits) {
+    // The only caller with try_bits passes grp_bits, so the row-list arm below never runs.  It stays because
+    // removing it shifts the register allocation of the short-vector kernels: on a B200 (1000 W, 1965 MHz),
+    // K2 got 1.1 % faster on the target, config 5 and config 2 but 0.15 % slower on config 1
+    // (0.2825 against 0.2821 ms per step, run-to-run spread 0.0001 ms).
+    if (grp_bits) {
       // the group's rows from its membership mask instead of its list: the rows that are also missing in the
       // other column (nab_other; most of x's missing rows at correlated missingness) have its lowest rank and
       // are only counted -- one popcount per word -- and only the others look their rank up
@@ -530,14 +525,12 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
 // walk equally far (in list order a group's rows walk t-1, t-2, ... 0 steps and half of the warp
 // idles).  One comparison for the usual isolated tie; K1 bounds the total (groups of kLargeTie rows
 // or more are only left to this routine while the sum of their size^2 stays below kDirectBudget * n).
-template <bool G, bool RG>
-__device__ __forceinline__ void small_groups_direct(typename Mem<G>::ptr keys, const int m,
+// Runs where y's rank table is staged in shared memory (short vectors); small_groups_inplace elsewhere.
+__device__ __forceinline__ void small_groups_direct(const uint32_t keys, const int m,
                                                     const uint16_t* __restrict__ trow,
                                                     const uint32_t* __restrict__ tord,
-                                                    typename Mem<G>::ptr rank_tbl,
-                                                    const uint16_t* __restrict__ rank_g, uint32_t& inv,
-                                                    uint32_t& ties) {
-  typedef Mem<G> M;
+                                                    const uint32_t rank_tbl, uint32_t& inv, uint32_t& ties) {
+  typedef Mem<false> M;
   const int tid = threadIdx.x, T = blockDim.x;
   // the first walk-order entry is fetched before the key gather, later ones one step ahead: the
   // global-load latency would otherwise sit between the barrier and the first comparison
@@ -552,8 +545,8 @@ __device__ __forceinline__ void small_groups_direct(typename Mem<G>::ptr keys, c
       for (int j = 0; j < 4; ++j) {
         const uint32_t r0 = pw[j] & 0xffffu, r1 = pw[j] >> 16;
         const bool v0 = (t8 << 3) + 2 * j < m, v1 = (t8 << 3) + 2 * j + 1 < m;  // rows behind m are stale
-        const uint32_t k0 = !v0 ? 0u : RG ? (uint32_t)__ldg(rank_g + r0) : M::ld16(M::add(rank_tbl, (int32_t)(r0 << 1)));
-        const uint32_t k1 = !v1 ? 0u : RG ? (uint32_t)__ldg(rank_g + r1) : M::ld16(M::add(rank_tbl, (int32_t)(r1 << 1)));
+        const uint32_t k0 = v0 ? M::ld16(M::add(rank_tbl, (int32_t)(r0 << 1))) : 0u;
+        const uint32_t k1 = v1 ? M::ld16(M::add(rank_tbl, (int32_t)(r1 << 1))) : 0u;
         o[j] = k0 | (k1 << 16);
       }
       M::st128(M::add(keys, t8 << 4), o[0], o[1], o[2], o[3]);
@@ -619,52 +612,19 @@ __device__ __forceinline__ void small_groups_inplace(typename Mem<G>::ptr seq, c
 // round: bin = (group in batch) * K + rank, as many groups per batch as the counter area holds; if
 // not even one group's K counters fit, one group at a time in windows of ranks.  Returns (summed
 // over the threads) the joint ties inside those groups.  `pre` is a shared array of 256 words;
-// `lg` the column's (start, size) table.
+// `lg` the column's (start, size) table.  Runs where y's rank table is staged in shared memory (short
+// vectors); large_groups_sorted2 elsewhere.
 // Rows of one bin met by several lanes are added once (match.any + one atomic per distinct bin).  Plain
-// shared-memory atomics (ICIKT_MATCH_DEDUP=0) are 3 % faster on config 4 (27.7 against 28.6 ms), but the
-// different register allocation of the whole kernel costs the tie-free target 2.7 % (278.9 against 271.4 ms,
-// same box clocks; profiles/r02_match_dedup_ab.txt), so the deduplicating form stays.
-#ifndef ICIKT_MATCH_DEDUP
-#define ICIKT_MATCH_DEDUP 1
-#endif
-constexpr bool kMatchDedup = ICIKT_MATCH_DEDUP != 0;
-// ICIKT_LG_FROM_SEQ: the histogram of a large group reads the y ranks back from the sequence (shared memory,
-// consecutive) instead of looking them up again through perm_x (0 never, 1 where the rank table is not
-// staged, 2 always).  ICIKT_LG_PLAIN_RG: plain atomics where the rank table is not staged.
-#ifndef ICIKT_LG_FROM_SEQ
-#define ICIKT_LG_FROM_SEQ 1
-#endif
-#ifndef ICIKT_LG_PLAIN_RG
-#define ICIKT_LG_PLAIN_RG 1
-#endif
-constexpr int kFromSeq = ICIKT_LG_FROM_SEQ, kPlainRG = ICIKT_LG_PLAIN_RG;
-// ICIKT_SMALL_INPLACE: where the rank table is not staged, small tie groups are compared on the gathered
-// sequence (small_groups_inplace) instead of on a second copy of the tied rows' keys
-#ifndef ICIKT_SMALL_INPLACE
-#define ICIKT_SMALL_INPLACE 1
-#endif
-constexpr bool kSmallInplace = ICIKT_SMALL_INPLACE != 0;
-// ICIKT_LG_V2: large_groups_sorted2 instead of large_groups_sorted (0 never, 1 where the rank table is not staged, 2 always)
-#ifndef ICIKT_LG_V2
-#define ICIKT_LG_V2 1
-#endif
-constexpr int kLgV2 = ICIKT_LG_V2;
-// ICIKT_STAGED_GATHER: the in-place variant stages y's rank table in parts through the idle counter area
-// (staged_gather) and sorts x's first group with the large groups (large_groups_sorted2)
-#ifndef ICIKT_STAGED_GATHER
-#define ICIKT_STAGED_GATHER 1
-#endif
-constexpr bool kStagedGather = ICIKT_STAGED_GATHER != 0;
-template <bool G, bool RG>
-__device__ __forceinline__ uint32_t large_groups_sorted(typename Mem<G>::ptr buf, typename Mem<G>::ptr hist,
-                                                        const int hist_words, const uint16_t* __restrict__ permX,
-                                                        typename Mem<G>::ptr rank_tbl,
-                                                        const uint16_t* __restrict__ rank_g, const int K,
-                                                        const uint16_t* __restrict__ lg, const int nlg,
+// shared-memory atomics are 3 % faster on config 4 (27.7 against 28.6 ms), but the different register
+// allocation of the whole kernel costs the tie-free target 2.7 % (278.9 against 271.4 ms, same box clocks;
+// profiles/r02_match_dedup_ab.txt), so the deduplicating form stays.
+__device__ __forceinline__ uint32_t large_groups_sorted(const uint32_t buf, const uint32_t hist, const int hist_words,
+                                                        const uint16_t* __restrict__ permX, const uint32_t rank_tbl,
+                                                        const int K, const uint16_t* __restrict__ lg, const int nlg,
                                                         uint32_t* __restrict__ pre, uint32_t* __restrict__ list,
                                                         const int list_cap, uint32_t* descT, uint32_t* list_n,
                                                         const int nwarps) {
-  typedef Mem<G> M;
+  typedef Mem<false> M;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, T = blockDim.x;
   const int bins_avail = 2 * hist_words;
   const int gb_max = max(1, min(255, bins_avail / K));  // groups per batch (pre[] holds 256 words)
@@ -693,25 +653,14 @@ __device__ __forceinline__ uint32_t large_groups_sorted(typename Mem<G>::ptr buf
           uint32_t bin = 0x80000000u | (uint32_t)lane;  // idle lanes: a key of their own
           bool in = false;
           if (q < t) {
-            uint32_t r;
-            if (kFromSeq >= (RG ? 1 : 2) && kw == K) {
-              // the gather has put rank_y[perm_x[s0 + q]] at position s0 + q of the sequence, and with all of
-              // y's ranks in one window nothing of this batch is rewritten before the barrier below
-              r = M::ld16(M::add(buf, (int32_t)((s0 + q) << 1)));
-            } else {
-              const uint32_t row = permX[s0 + q];
-              r = (RG ? (uint32_t)__ldg(rank_g + row) : M::ld16(M::add(rank_tbl, (int32_t)(row << 1)))) - (uint32_t)k0;
-            }
+            const uint32_t row = permX[s0 + q];
+            const uint32_t r = M::ld16(M::add(rank_tbl, (int32_t)(row << 1))) - (uint32_t)k0;
             in = r < (uint32_t)kw;
             if (in) bin = (uint32_t)(j * kw) + r;
           }
-          if (kMatchDedup && (kPlainRG == 0 || !RG)) {  // rows of one bin met by several lanes are added once
-            const uint32_t peers = __match_any_sync(FULL, bin);
-            if (in && (peers & ((1u << lane) - 1u)) == 0u)
-              M::red_add32(M::add(hist, (int32_t)((bin >> 1) << 2)), (uint32_t)__popc(peers) << ((bin & 1u) * 16u));
-          } else if (in) {
-            M::red_add32(M::add(hist, (int32_t)((bin >> 1) << 2)), 1u << ((bin & 1u) * 16u));
-          }
+          const uint32_t peers = __match_any_sync(FULL, bin);
+          if (in && (peers & ((1u << lane) - 1u)) == 0u)
+            M::red_add32(M::add(hist, (int32_t)((bin >> 1) << 2)), (uint32_t)__popc(peers) << ((bin & 1u) * 16u));
         }
       }
       __syncthreads();
@@ -789,8 +738,11 @@ __device__ __forceinline__ uint32_t large_groups_sorted(typename Mem<G>::ptr buf
   return ties;
 }
 
-// Second form of large_groups_sorted, used where ICIKT_LG_V2 selects it (long vectors: rank table not
-// staged).  Same rounds and counters; what differs is everything around them:
+// Second form of large_groups_sorted, used where y's rank table is not staged in shared memory (long vectors:
+// the global-scratch and in-place variants).  Same rounds and counters; what differs is everything around them:
+//   * with all of y's ranks in one window, a row's rank is read back from the sequence, where the gather has
+//     put rank_y[perm_x[s0 + q]] at position s0 + q (nothing of the batch is rewritten before the barrier
+//     that ends the histogram), instead of being looked up again through perm_x;
 //   * the batch's (start, size) pairs are fetched once by nb threads into shared memory and warp 0 turns them
 //     into the output slot of each group's first counter (instead of one thread walking the global table, and
 //     a global load per non-empty counter in the emission);
@@ -799,17 +751,10 @@ __device__ __forceinline__ uint32_t large_groups_sorted(typename Mem<G>::ptr buf
 //   * runs of kListRun (16) keys and more are parked in the list, longer ones in pieces of kRunPiece, and every
 //     list entry is written by one warp (the CTA-wide loop spent 28 loop headers per entry).
 // `pre` = 256 words of shared memory: [0,128) the packed group table, [128,256) the output slots.
-#ifndef ICIKT_WIDE_GROUP
-#define ICIKT_WIDE_GROUP 512
-#endif
-#ifndef ICIKT_LIST_RUN
-#define ICIKT_LIST_RUN 16
-#endif
-constexpr int kWideGroup = ICIKT_WIDE_GROUP, kListRun = ICIKT_LIST_RUN, kRunPiece = 512;
-template <bool G, bool RG>
+constexpr int kWideGroup = 512, kListRun = 16, kRunPiece = 512;
+template <bool G>
 __device__ __forceinline__ uint32_t large_groups_sorted2(typename Mem<G>::ptr buf, typename Mem<G>::ptr hist,
                                                          const int hist_words, const uint16_t* __restrict__ permX,
-                                                         typename Mem<G>::ptr rank_tbl,
                                                          const uint16_t* __restrict__ rank_g, const int K,
                                                          const uint16_t* __restrict__ lg, const int nlg,
                                                          uint32_t* __restrict__ pre, uint32_t* __restrict__ list,
@@ -866,11 +811,11 @@ __device__ __forceinline__ uint32_t large_groups_sorted2(typename Mem<G>::ptr bu
       // 1. histogram
       auto add_row = [&](const int j, const int s0, const int q) {
         uint32_t r;
-        if (RG && kw == K) {  // the gather has put rank_y[perm_x[s0 + q]] there, see large_groups_sorted
+        if (kw == K) {  // the gather has put rank_y[perm_x[s0 + q]] there
           r = M::ld16(M::add(buf, (int32_t)((s0 + q) << 1)));
         } else {
           const uint32_t row = permX[s0 + q];
-          r = (RG ? (uint32_t)__ldg(rank_g + row) : M::ld16(M::add(rank_tbl, (int32_t)(row << 1)))) - (uint32_t)k0;
+          r = (uint32_t)__ldg(rank_g + row) - (uint32_t)k0;
         }
         if (r < (uint32_t)kw) {
           const uint32_t bin = (uint32_t)(j * kw) + r;
@@ -887,11 +832,11 @@ __device__ __forceinline__ uint32_t large_groups_sorted2(typename Mem<G>::ptr bu
             const int q = qw + lane;
             uint32_t r = 0xffffffffu;
             if (q < t) {
-              if (RG && kw == K) {
+              if (kw == K) {
                 r = M::ld16(M::add(buf, (int32_t)(q << 1)));
               } else {
                 const uint32_t row = permX[q];
-                r = RG ? (uint32_t)__ldg(rank_g + row) : M::ld16(M::add(rank_tbl, (int32_t)(row << 1)));
+                r = (uint32_t)__ldg(rank_g + row);
               }
             }
             zeros += __popc(__ballot_sync(FULL, r == 0u));
@@ -1167,7 +1112,7 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
   constexpr bool RG = G || IP != 0;    // rank table not staged
   constexpr int AQ = IP != 0 ? 2 : 4;  // bytes of the pass-A buffers in units of cap
   // in place: the rank table passes through the counter area in parts, the first group is sorted with the large ones
-  constexpr bool STG = IP != 0 && kStagedGather && kLgV2 >= 1;
+  constexpr bool STG = IP != 0;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int T = blockDim.x, nwarps = T >> 5;
@@ -1274,9 +1219,11 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
       const int m = XS.n_tied, nlg = XS.flags >> 8;
       const bool by_pass_b = nlg > 0 && p.tier == 2 && (long long)nlg * YS.n_groups > p.budget;
       uint32_t accB = 0;
-      if (!(RG && kSmallInplace) && m > 0 && !by_pass_b)  // keys: 2 m <= 2 cap bytes, the still empty sequence buffer
-        small_groups_direct<G, RG>(bufA, m, p.trow + (size_t)xcol * p.nstride, p.tord + (size_t)xcol * p.nstride,
-                                   rank_tbl, rankY_g, accB, ties);
+      if constexpr (!RG) {
+        if (m > 0 && !by_pass_b)  // keys: 2 m <= 2 cap bytes, the still empty sequence buffer
+          small_groups_direct(bufA, m, p.trow + (size_t)xcol * p.nstride, p.tord + (size_t)xcol * p.nstride,
+                              rank_tbl, accB, ties);
+      }
       // x's first tie group goes in already sorted by y; its joint ties with y fall out of it
       if (!STG && f > 0) {
         if (PW && XS.n_na > 0)
@@ -1330,20 +1277,20 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
         }
       }
       __syncthreads();
-      if (RG && kSmallInplace && m > 0 && !by_pass_b)
+      if (RG && m > 0 && !by_pass_b)
         small_groups_inplace<G>(bufA, m, p.tord + (size_t)xcol * p.nstride, p.tpos + (size_t)xcol * p.nstride, accB, ties);
       if ((nlg > 0 || (STG && f > 0)) && !by_pass_b) {
         // large tie groups of x: sorted by y in place (the counters live behind the two pass-A buffers)
-        if (kLgV2 >= (RG ? 1 : 2))
-          ties += large_groups_sorted2<G, RG>(bufA, M::add(bufA, AQ * cap), (p.region_bytes - AQ * cap) >> 2, permX, rank_tbl, rankY_g, YS.n_groups,
-                                              p.lgrp + (size_t)xcol * kLargeStride, nlg,
-                                              reinterpret_cast<uint32_t*>(sm.red), sm.fmask, fmask_words(nwarps, kkc) / 3,
-                                              sm.descT, sm.mini + 16, nwarps, STG ? f : 0, sm.mini + 18);
+        if constexpr (RG)
+          ties += large_groups_sorted2<G>(bufA, M::add(bufA, AQ * cap), (p.region_bytes - AQ * cap) >> 2, permX, rankY_g, YS.n_groups,
+                                          p.lgrp + (size_t)xcol * kLargeStride, nlg,
+                                          reinterpret_cast<uint32_t*>(sm.red), sm.fmask, fmask_words(nwarps, kkc) / 3,
+                                          sm.descT, sm.mini + 16, nwarps, STG ? f : 0, sm.mini + 18);
         else
-        ties += large_groups_sorted<G, RG>(bufA, M::add(bufA, AQ * cap), (p.region_bytes - AQ * cap) >> 2, permX, rank_tbl, rankY_g, YS.n_groups,
-                                       p.lgrp + (size_t)xcol * kLargeStride, nlg,
-                                       reinterpret_cast<uint32_t*>(sm.red), sm.fmask, fmask_words(nwarps, kkc) / 3,
-                                       sm.descT, sm.mini + 16, nwarps);
+          ties += large_groups_sorted(bufA, M::add(bufA, AQ * cap), (p.region_bytes - AQ * cap) >> 2, permX, rank_tbl, YS.n_groups,
+                                      p.lgrp + (size_t)xcol * kLargeStride, nlg,
+                                      reinterpret_cast<uint32_t*>(sm.red), sm.fmask, fmask_words(nwarps, kkc) / 3,
+                                      sm.descT, sm.mini + 16, nwarps);
       }
       unsigned long long accA = 0;
       const uint32_t lead = sm.mini[18];  // published by the barrier after the gather
