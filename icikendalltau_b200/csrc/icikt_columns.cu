@@ -665,11 +665,8 @@ __global__ void __launch_bounds__(SORT_THREADS)
     unsigned long long acc = 0;
     if ((tid >> 5) < nw) {
       count_pass<false>(bufA, bufB, 1, nw, L, descA, descB, tid & 31, tid >> 5, pc, acc);
-    } else {  // count_pass has two block-wide barriers per two-bit level
-      for (int lv = (L - 1) & ~1; lv >= 0; lv -= 2) {
-        __syncthreads();
-        __syncthreads();
-      }
+    } else {
+      for (int b = count_pass_barriers(L); b > 0; --b) __syncthreads();
     }
     const long long total = block_sum_ll((long long)acc, llbuf);
     if (tid == 0) stats[col].cconst = (uint64_t)total;

@@ -50,6 +50,23 @@ __host__ __device__ inline PipeConst make_pipe_const() {
   return pc;
 }
 
+// Pass A's low-nibble level (count_pass, after the two-bit levels down to bit 4).  For a key with low
+// nibble b3 b2 b1 b0, the four one-bit levels below bit 4 add, at every bit whose value is 0, the keys
+// before it that agree with it on the nibble's higher bits and have that bit set: a binary tree of 15
+// nodes.  Earlier buckets and the other subtrees only add terms that depend on column y alone (cconst
+// takes them), so ONE sweep over the order the last two-bit level left counts all four bits, and
+// nothing has to be stored.  A thread keeps the counts of its range's keys seen so far in byte fields
+// (a range holds R = 8 kk <= 255 keys):
+//   C    keys per class (b3 b2)            root: c2 + c3 ones, node b3: c(2 b3 + 1) ones
+//   D2   ones of b1 per (b3 b2)
+//   D3a  ones of b0 per (b2 b1), b3 = 0;  D3b the same for b3 = 1
+// Every key adds, unpredicated, the ones counters of the four nodes on its path (one dp4a per register,
+// C with byte weights 0,1,1,1 or 0,0,1,2); the keys with bit 1 at a node add C(n1, 2) there in all,
+// which nibble_level takes back out in closed form.
+struct NibbleCounts {
+  uint32_t C, D2, D3a, D3b, acc;
+};
+
 // ---- TMA bulk copy global -> shared, completion on an mbarrier (sm_90+) ---------------------
 // Used for the one contiguous bulk transfer of the pair kernel: y's dense-rank table into the
 // second sequence buffer.  One thread issues it; the copy engine moves the bytes while the CTA
@@ -152,25 +169,35 @@ struct Mem<false> {
           "r"(pc.c4410), "r"(pc.c4432), "r"(pc.one)
         : "memory");
   }
-  // the same without the store: the last level only has to count
-  static __device__ __forceinline__ void step4c(uint32_t& Q01, uint32_t& Q23, uint32_t& acc2, uint32_t w,
-                                                uint32_t bit_lo, uint32_t bit_hi, const PipeConst& pc) {
+  // one key of the low-nibble level (see NibbleCounts): the key's nibble sits at bit SH of w, a2 / a3 hold
+  // 8*(b3 b2) / 8*(b2 b1) in their low five bits (a shift by a register uses those only).  ~16 instructions.
+  template <int SH>
+  static __device__ __forceinline__ void step16(NibbleCounts& s, uint32_t w, uint32_t a2, uint32_t a3) {
     asm volatile(
         "{\n\t"
-        ".reg .pred ph, pl;\n\t"
-        ".reg .b32 t, qs, inc;\n\t"
-        "and.b32 t, %3, %5;\n\t"
-        "setp.ne.u32 ph, t, 0;\n\t"
-        "and.b32 t, %3, %4;\n\t"
-        "setp.ne.u32 pl, t, 0;\n\t"
-        "selp.b32 qs, %1, %0, ph;\n\t"
-        "mad.hi.u32 %2, qs, %6, %2;\n\t"
-        "selp.b32 inc, %6, %7, pl;\n\t"
-        "@ph add.u32 %1, %1, inc;\n\t"
-        "@!ph add.u32 %0, %0, inc;\n\t"
+        ".reg .pred p3, p1, p0;\n\t"
+        ".reg .b32 t, W1, W2, W3, Ds;\n\t"
+        "and.b32 t, %5, %8;\n\t"
+        "setp.ne.u32 p3, t, 0;\n\t"
+        "and.b32 t, %5, %9;\n\t"
+        "setp.ne.u32 p1, t, 0;\n\t"
+        "and.b32 t, %5, %10;\n\t"
+        "setp.ne.u32 p0, t, 0;\n\t"
+        "selp.b32 W1, 0x02010000, 0x01010100, p3;\n\t"
+        "dp4a.u32.u32 %4, %0, W1, %4;\n\t"
+        "shf.l.wrap.b32 W2, 0, 1, %6;\n\t"
+        "add.u32 %0, %0, W2;\n\t"
+        "dp4a.u32.u32 %4, %1, W2, %4;\n\t"
+        "@p1 add.u32 %1, %1, W2;\n\t"
+        "shf.l.wrap.b32 W3, 0, 1, %7;\n\t"
+        "selp.b32 Ds, %3, %2, p3;\n\t"
+        "dp4a.u32.u32 %4, Ds, W3, %4;\n\t"
+        "selp.b32 W3, W3, 0, p0;\n\t"
+        "@p3 add.u32 %3, %3, W3;\n\t"
+        "@!p3 add.u32 %2, %2, W3;\n\t"
         "}"
-        : "+r"(Q01), "+r"(Q23), "+r"(acc2)
-        : "r"(w), "r"(bit_lo), "r"(bit_hi), "r"(pc.c64k), "r"(pc.one));
+        : "+r"(s.C), "+r"(s.D2), "+r"(s.D3a), "+r"(s.D3b), "+r"(s.acc)
+        : "r"(w), "r"(a2), "r"(a3), "n"(8u << SH), "n"(2u << SH), "n"(1u << SH));
   }
   static __device__ __forceinline__ void red_add32(ptr p, uint32_t v) {
     asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(p), "r"(v) : "memory");
@@ -216,13 +243,18 @@ struct Mem<true> {
     if (ph) Q23 += inc; else Q01 += inc;
     acc2 += qs >> 16;
   }
-  static __device__ __forceinline__ void step4c(uint32_t& Q01, uint32_t& Q23, uint32_t& acc2, uint32_t w,
-                                                uint32_t bit_lo, uint32_t bit_hi, const PipeConst&) {
-    const bool ph = (w & bit_hi) != 0u, pl = (w & bit_lo) != 0u;
-    const uint32_t qs = ph ? Q23 : Q01;
-    const uint32_t inc = pl ? 0x10000u : 1u;
-    if (ph) Q23 += inc; else Q01 += inc;
-    acc2 += qs >> 16;
+  template <int SH>
+  static __device__ __forceinline__ void step16(NibbleCounts& s, uint32_t w, uint32_t a2, uint32_t a3) {
+    const bool p3 = (w >> SH) & 8u, p1 = (w >> SH) & 2u, p0 = (w >> SH) & 1u;
+    s.acc = __dp4a(s.C, p3 ? 0x02010000u : 0x01010100u, s.acc);
+    const uint32_t W2 = 1u << (a2 & 31u), W3 = 1u << (a3 & 31u);
+    s.C += W2;
+    s.acc = __dp4a(s.D2, W2, s.acc);
+    if (p1) s.D2 += W2;
+    s.acc = __dp4a(p3 ? s.D3b : s.D3a, W3, s.acc);
+    if (p0) {
+      if (p3) s.D3b += W3; else s.D3a += W3;
+    }
   }
   static __device__ __forceinline__ void red_add32(ptr p, uint32_t v) { atomicAdd(reinterpret_cast<uint32_t*>(p), v); }
   static __device__ __forceinline__ uint32_t atom_or32(ptr p, uint32_t v) { return atomicOr(reinterpret_cast<uint32_t*>(p), v); }
@@ -258,7 +290,8 @@ struct Mem<true> {
 //            key's lo = 1 sibling class over all keys (step4); the lo = 1 keys' own share of that
 //            sum -- their destination slots, two arithmetic series -- is taken out in closed form.
 // No ballots, no per-key population counts: about 16 instructions per key and level of two bits.
-// With an odd number of bits the first level treats the missing top bit as zero.
+// With an odd number of bits the first level treats the missing top bit as zero.  The two-bit levels
+// stop at bit 4; the low four bits take one count-only sweep (NibbleCounts, nibble_level).
 //   acc64 += the count over all levels (this thread's share)
 struct LevelCounts {
   uint32_t n1, n2, n3, J1;
@@ -287,11 +320,82 @@ __device__ __forceinline__ uint32_t level_share(const LevelCounts& c, uint32_t R
   return hi_term + lo_term;
 }
 
+// the low-nibble sweep over one 32-bit word (two keys, the low one first)
+template <bool G>
+__device__ __forceinline__ void nibble_word(NibbleCounts& s, uint32_t w) {
+  const uint32_t a2 = (w << 1) & 0x00180018u, a3 = (w << 2) & 0x00180018u;
+  Mem<G>::template step16<0>(s, w, a2, a3);
+  Mem<G>::template step16<16>(s, w, a2 >> 16, a3 >> 16);
+}
+
+// The low-nibble level after its sweep: this thread's share is
+//   acc - sum over nodes of C(n1, 2)                    (within the range)
+//   + sum over nodes of n0 * (ones at the node in earlier ranges)
+// The 15 ones counts go through one warp scan as 16-bit pairs; lane 31 leaves the warp's totals in the
+// first 32 bytes of the warp's part of `a` (its keys are read and are not needed afterwards), where the
+// later warps add them after the barrier.  Two block-wide barriers.
+template <bool G>
+__device__ __forceinline__ void nibble_level(const NibbleCounts& s, const uint32_t R, const bool idle, const int lane,
+                                             const int warp, typename Mem<G>::ptr a, unsigned long long& acc64) {
+  typedef Mem<G> M;
+  const uint32_t warp_bytes = R << 6;
+  const uint32_t r = ((s.C >> 16) & 0xffu) + (s.C >> 24);  // ones at the root
+  const uint32_t q[8] = {__byte_perm(s.C, 0u, 0x4341),   r,
+                         __byte_perm(s.D2, 0u, 0x4140),  __byte_perm(s.D2, 0u, 0x4342),
+                         __byte_perm(s.D3a, 0u, 0x4140), __byte_perm(s.D3a, 0u, 0x4342),
+                         __byte_perm(s.D3b, 0u, 0x4140), __byte_perm(s.D3b, 0u, 0x4342)};
+  uint32_t incl[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) incl[k] = q[k];
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      const uint32_t t = __shfl_up_sync(FULL, incl[k], d);
+      if (lane >= d) incl[k] += t;
+    }
+  }
+  __syncwarp();
+  if (lane == 31) {
+    const typename M::ptr mine = M::add(a, (int32_t)((uint32_t)warp * warp_bytes));
+    M::st128(mine, incl[0], incl[1], incl[2], incl[3]);
+    M::st128(M::add(mine, 16), incl[4], incl[5], incl[6], incl[7]);
+  }
+  __syncthreads();
+  uint32_t v[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
+  if (lane < warp) {
+    const typename M::ptr o = M::add(a, (int32_t)((uint32_t)lane * warp_bytes));
+    M::ld128(o, v[0], v[1], v[2], v[3]);
+    M::ld128(M::add(o, 16), v[4], v[5], v[6], v[7]);
+  }
+  uint32_t E[8];  // ones before the range (exclusive prefix over the CTA; below 65 536)
+#pragma unroll
+  for (int k = 0; k < 8; ++k) E[k] = __reduce_add_sync(FULL, v[k]) + incl[k] - q[k];
+  if (!idle) {
+    // zeros per node: b1 = 0 per (b3 b2), then b0 = 0 per (b3 b2 b1) (bytewise, no borrows)
+    const uint32_t N2 = s.C - s.D2;
+    const uint32_t N3a = __byte_perm(N2, s.D2, 0x5140) - s.D3a, N3b = __byte_perm(N2, s.D2, 0x7362) - s.D3b;
+    uint32_t x = (R - r) * E[1];
+    x = __dp2a_lo(E[0], __byte_perm(s.C, 0u, 0x4420), x);  // c0 * E(c1) + c2 * E(c3)
+    x = __dp2a_hi(E[3], N2, __dp2a_lo(E[2], N2, x));
+    x = __dp2a_hi(E[5], N3a, __dp2a_lo(E[4], N3a, x));
+    x = __dp2a_hi(E[7], N3b, __dp2a_lo(E[6], N3b, x));
+    // sum of C(n1, 2) = (sum n1^2 - sum n1) / 2 over the 15 nodes
+    const uint32_t sq = __dp4a(s.D2, s.D2, __dp4a(s.D3a, s.D3a, __dp4a(s.D3b, s.D3b, __dp4a(s.C & 0xff00ff00u, s.C, r * r))));
+    const uint32_t li = __dp4a(s.D2, 0x01010101u, __dp4a(s.D3a, 0x01010101u, __dp4a(s.D3b, 0x01010101u, __dp4a(s.C, 0x01000100u, r))));
+    acc64 += (unsigned long long)(s.acc + x - ((sq - li) >> 1));
+  }
+  __syncthreads();  // the warp totals are read before anybody reuses the buffer
+}
+
+// block-wide barriers count_pass executes for L bits (threads that skip it must keep them)
+__host__ __device__ constexpr int count_pass_barriers(int L) { return 2 * (L > 4 ? ((L - 1) >> 1) : 1); }
+
 // `lead`: the sequence is known to START with that many zero keys (x's first tie group is written in
 // ascending y order, so its rows of y's lowest rank -- on left-censored data the rows missing in BOTH
 // columns, a fifth of all rows -- come first).  Zero keys are class 0 at every level and the stable
 // partition keeps a leading block of them exactly where it is; no one-key ever precedes them, so they
-// add nothing to any count.  Threads whose whole range lies inside that block skip both sweeps of
+// add nothing to any count.  Threads whose whole range lies inside that block skip the sweeps of
 // every level (they only take part in the scans, with zero counts, and in the barriers).
 template <bool G>
 __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<G>::ptr b, const int kk,
@@ -305,11 +409,11 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
   const uint32_t my_pos = tid * R;
   const uint32_t cap = ((uint32_t)nwarps << 5) * R;    // keys per buffer
   const bool idle = my_pos + R <= lead;
-  if (idle && L > 2) {  // the block must read as zeros in the other buffer too (levels alternate)
+  if (idle && L > 4) {  // the block must read as zeros in the other buffer too (levels alternate)
     const typename M::ptr rb = M::add(b, (int32_t)my_off);
     for (int c = 0; c < kk; ++c) M::st128(M::add(rb, c << 4), 0u, 0u, 0u, 0u);
   }
-  for (int s = (L - 1) & ~1; s >= 0; s -= 2) {
+  for (int s = (L - 1) & ~1; s >= 4; s -= 2) {
     const typename M::ptr ra = M::add(a, (int32_t)my_off);
     uint32_t cl = 0, cb = 0, wm = 0, m4 = 0;
     uint32_t chj[4] = {0u, 0u, 0u, 0u};
@@ -361,7 +465,7 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     asm volatile("" : "+r"(bLl), "+r"(bHl), "+r"(bLh), "+r"(bHh));  // keep the bit tests single LOP3s
     if (idle) {
       // nothing to move, nothing to count
-    } else if (s > 0) {
+    } else {
 #pragma unroll 1
       for (int c = 0; c < kk; ++c) {
         uint32_t w[4];
@@ -372,17 +476,6 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
           M::step4(Q01, Q23, acc2, w[j], bLh, bHh, M::hi16(w[j], pc.c64k), b, pc);
         }
       }
-    } else {  // the sorted sequence itself is not needed: the last level only counts
-#pragma unroll 1
-      for (int c = 0; c < kk; ++c) {
-        uint32_t w[4];
-        M::ld128(M::add(ra, c << 4), w[0], w[1], w[2], w[3]);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          M::step4c(Q01, Q23, acc2, w[j], bLl, bHl, pc);
-          M::step4c(Q01, Q23, acc2, w[j], bLh, bHh, pc);
-        }
-      }
     }
     (void)N3;
     if (!idle) acc64 += (unsigned long long)level_share(lc, R, acc2, e2 + e3, start1, start3, N0, N2);
@@ -391,6 +484,16 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     a = b;
     b = t;
   }
+  NibbleCounts nc = {0u, 0u, 0u, 0u, 0u};
+  const typename M::ptr ra = M::add(a, (int32_t)my_off);
+#pragma unroll 1
+  for (int c = 0; c < (idle ? 0 : kk); ++c) {
+    uint32_t w[4];
+    M::ld128(M::add(ra, c << 4), w[0], w[1], w[2], w[3]);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) nibble_word<G>(nc, w[j]);
+  }
+  nibble_level<G>(nc, R, idle, lane, warp, a, acc64);
 }
 
 }  // namespace

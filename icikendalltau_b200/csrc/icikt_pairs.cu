@@ -19,7 +19,7 @@
 //   level, lane-sequential: thread t owns a contiguous range of the sequence, counts its keys per
 //   digit class with SIMD-in-a-word adds, two packed warp scans give the class offsets, then the
 //   thread walks its range with four running slot indices and scatters the keys (STS.U16).  No
-//   ballots and no per-key popc.  Because every row is present, the bucket layout (keys agreeing
+//   ballots and no per-key popc.  The low four bits take one count-only level that stores nothing.  Because every row is present, the bucket layout (keys agreeing
 //   on the higher bits) and the number of ones before each bucket are properties of column y
 //   alone, so the per-bucket offsets collapse into one per-column constant `cconst` (the raw
 //   count of y's own sorted sequence, which has no inversions; computed by K1):
@@ -186,7 +186,7 @@ __device__ __forceinline__ void count_pass_inplace(const uint32_t a, const int n
   const uint32_t cap = ((uint32_t)nwarps << 5) * R;
   const uint32_t ra = a + my_off;
   const bool idle = my_pos + R <= lead;  // inside the leading block of zero keys, see count_pass
-  for (int s = (L - 1) & ~1; s >= 0; s -= 2) {
+  for (int s = (L - 1) & ~1; s >= 4; s -= 2) {
     uint32_t w[KK][4];
     uint32_t cl = 0, ch = 0, cb = 0, wm = 0;
     if (idle) {  // (block-divergent, warp-mostly-uniform) nothing to load: every key is zero
@@ -235,9 +235,7 @@ __device__ __forceinline__ void count_pass_inplace(const uint32_t a, const int n
     uint32_t acc2 = 0;
     uint32_t bLl = 1u << s, bHl = 2u << s, bLh = 1u << (s + 16), bHh = 2u << (s + 16);
     asm volatile("" : "+r"(bLl), "+r"(bHl), "+r"(bLh), "+r"(bHh));
-    if (idle) {
-      // the block stays where it is
-    } else if (s > 0) {
+    if (!idle) {  // (idle: the block stays where it is)
 #pragma unroll
       for (int c = 0; c < KK; ++c) {
 #pragma unroll
@@ -246,20 +244,23 @@ __device__ __forceinline__ void count_pass_inplace(const uint32_t a, const int n
           M::step4(Q01, Q23, acc2, w[c][j], bLh, bHh, M::hi16(w[c][j], pc.c64k), a, pc);
         }
       }
-    } else {
-#pragma unroll
-      for (int c = 0; c < KK; ++c) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          M::step4c(Q01, Q23, acc2, w[c][j], bLl, bHl, pc);
-          M::step4c(Q01, Q23, acc2, w[c][j], bLh, bHh, pc);
-        }
-      }
     }
     (void)N3;
     if (!idle) acc64 += (unsigned long long)level_share(lc, R, acc2, e2 + e3, start1, start3, N0, N2);
     __syncthreads();
   }
+  // the low nibble, as in count_pass (the sweep writes nothing, so the keys need not stay in registers)
+  NibbleCounts nc = {0u, 0u, 0u, 0u, 0u};
+  if (!idle) {
+#pragma unroll
+    for (int c = 0; c < KK; ++c) {
+      uint32_t w[4];
+      M::ld128(ra + (c << 4), w[0], w[1], w[2], w[3]);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) nibble_word<false>(nc, w[j]);
+    }
+  }
+  nibble_level<false>(nc, R, idle, lane, warp, a, acc64);
 }
 
 // Per-thread sums of the complete-observations mode for one side of a pair (see group_hist).
@@ -1756,9 +1757,8 @@ int measure_issue_rate(double* alu, double* fma, double* mixed) {
   return 0;
 }
 
-// Pass A sums the word indices of a thread's hi = 1 keys in two packed 16-bit fields (count_pass):
-// 2 kk (4 kk - 1) must stay below 65 536
-constexpr int kMaxRuns = 90;
+// Pass A's low-nibble level counts a thread's 8 kk keys in byte fields (NibbleCounts): 8 kk <= 255
+constexpr int kMaxRuns = 31;
 
 // 8-key runs per thread such that W warps cover n keys: the smallest odd count (bank-conflict-free
 // 128-bit loads), unless that pushes the padded length past the 65536 slots the packed 16-bit
