@@ -33,6 +33,8 @@ EXPORTS = [
     "icikt_pairwise_completeness", "icikt_plan_upload_columns", "icikt_plan_columns_range",
     "icikt_plan_tables", "icikt_plan_columns_finish", "icikt_measure_issue_rate",
     "icikt_matrices_multi", "icikt_stage_table", "icikt_launch_shape",
+    "icikt_all_pairs_csc", "icikt_all_pairs_multi_csc", "icikt_pair_list_csc", "icikt_matrices_csc",
+    "icikt_matrices_multi_csc", "icikt_pairwise_completeness_csc",
 ]
 NSTATUS = 10
 
@@ -142,6 +144,13 @@ def load():
                                               ctypes.c_int32, ctypes.c_int32, _ip, _ip, ctypes.c_int64, _ip,
                                               _dp, _dp]
     L.icikt_pairwise_completeness.restype = ctypes.c_int
+    # the *_csc twins: (data, n, C, ld) -> (colptr, rowidx, values, n, C)
+    csc = [_lp, _ip, _dp, ctypes.c_int64, ctypes.c_int64]
+    for name in ("icikt_all_pairs", "icikt_all_pairs_multi", "icikt_pair_list", "icikt_matrices",
+                 "icikt_matrices_multi", "icikt_pairwise_completeness"):
+        f = getattr(L, name + "_csc")
+        f.argtypes = csc + getattr(L, name).argtypes[4:]
+        f.restype = ctypes.c_int
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -195,19 +204,70 @@ def _ptr(a, t=None):
     return a.__array_interface__["data"][0] if a is not None else None
 
 
+def is_sparse(x):
+    """True for a scipy.sparse matrix or array (scipy is imported only for objects that may be one)."""
+    if not hasattr(x, "tocsc"):
+        return False
+    import scipy.sparse as sp
+    return sp.issparse(x)
+
+
+def canonical_csc(x):
+    """x as a scipy.sparse CSC matrix or array in canonical format (rows sorted and unique within each
+    column).  Duplicate entries are summed, as toarray() does, on a copy: the caller's object stays as it is."""
+    a = x.tocsc()
+    if len(a.shape) != 2:
+        raise ValueError("data must be a 2-D array (features x samples)")
+    if not a.has_canonical_format:
+        a = a.copy()
+        a.sum_duplicates()
+    return a
+
+
+class CSC:
+    """A sparse matrix as the *_csc entry points take it: colptr int64 [C + 1], rowidx int32 and values
+    float64 [nnz] of its canonical CSC form.  Entries not stored are 0.0."""
+
+    def __init__(self, x):
+        a = canonical_csc(x)
+        self.shape = (int(a.shape[0]), int(a.shape[1]))
+        self.colptr = np.ascontiguousarray(a.indptr, dtype=np.int64)
+        self.rowidx = np.ascontiguousarray(a.indices, dtype=np.int32)
+        self.values = np.ascontiguousarray(a.data, dtype=np.float64)
+        nnz = int(self.colptr[-1]) if self.colptr.size else 0
+        if self.colptr.size != self.shape[1] + 1 or self.rowidx.size != nnz or self.values.size != nnz:
+            raise ValueError(f"malformed CSC matrix: {self.colptr.size} column pointers for {self.shape[1]} columns, "
+                             f"colptr[C] = {nnz}, {self.rowidx.size} row indices, {self.values.size} values")
+
+    def args(self):
+        """the leading (colptr, rowidx, values, n, C) arguments of a *_csc entry point"""
+        return (_ptr(self.colptr), _ptr(self.rowidx), _ptr(self.values)) + self.shape
+
+
+def _matrix_args(data):
+    """(leading arguments of the dense or the *_csc entry point, suffix of its name, n, C, the object that
+    owns the memory those arguments point into)"""
+    if is_sparse(data):
+        m = CSC(data)
+        return m.args(), "_csc", m.shape[0], m.shape[1], m
+    data = np.asfortranarray(data, dtype=np.float64)
+    if data.ndim != 2:
+        raise ValueError("data must be a 2-D array (features x samples)")
+    n, C = data.shape
+    return (_ptr(data, _dp), n, C, n), "", n, C, data
+
+
 def run_pairs(data, global_na=(), pi=None, pj=None, want_counts=False, devices=None, **opt_kw):
     """One-shot call through icikt_all_pairs / icikt_pair_list with host buffers.
 
-    data: (n, C) array (copied to Fortran order if needed).  Returns a dict of NumPy arrays in
+    data: (n, C) array (copied to Fortran order if needed), or a scipy.sparse matrix (-> the *_csc entry
+    points; entries not stored are 0.0).  Returns a dict of NumPy arrays in
     pair order: raw, pvalue, taumax, completeness, status, [counts], max_taumax, timings.
     devices: list of CUDA ordinals -> icikt_all_pairs_multi (all pairs only): every device takes a
     contiguous slice of the pair order.
     """
     L = load()
-    data = np.asfortranarray(data, dtype=np.float64)
-    if data.ndim != 2:
-        raise ValueError("data must be a 2-D array (features x samples)")
-    n, C = data.shape
+    lead, sfx, n, C, keep_alive = _matrix_args(data)
     o = make_opts(want_counts=want_counts, **opt_kw)
     if pi is None:
         ptot = C * (C - 1) // 2 + (C if o.include_diag else 0)
@@ -230,16 +290,16 @@ def run_pairs(data, global_na=(), pi=None, pj=None, want_counts=False, devices=N
     g, gp, ng = _global_na_array(global_na)
     if pi is None and devices is not None:
         dev = np.ascontiguousarray(list(devices), dtype=np.int32)
-        rc = L.icikt_all_pairs_multi(_ptr(data, _dp), n, C, n, gp, ng, ctypes.byref(o), _ptr(dev, _ip),
-                                     int(dev.size), a_raw, a_pv, a_tm, a_comp, a_status, _ptr(counts, _lp),
-                                     ctypes.byref(mx), ctypes.byref(t))
+        rc = getattr(L, "icikt_all_pairs_multi" + sfx)(*lead, gp, ng, ctypes.byref(o), _ptr(dev, _ip),
+                                                       int(dev.size), a_raw, a_pv, a_tm, a_comp, a_status,
+                                                       _ptr(counts, _lp), ctypes.byref(mx), ctypes.byref(t))
     elif pi is None:
-        rc = L.icikt_all_pairs(_ptr(data, _dp), n, C, n, gp, ng, ctypes.byref(o), a_raw, a_pv, a_tm, a_comp,
-                               a_status, _ptr(counts, _lp), ctypes.byref(mx), ctypes.byref(t))
+        rc = getattr(L, "icikt_all_pairs" + sfx)(*lead, gp, ng, ctypes.byref(o), a_raw, a_pv, a_tm, a_comp,
+                                                 a_status, _ptr(counts, _lp), ctypes.byref(mx), ctypes.byref(t))
     else:
-        rc = L.icikt_pair_list(_ptr(data, _dp), n, C, n, gp, ng, _ptr(pi, _ip), _ptr(pj, _ip), P,
-                               ctypes.byref(o), a_raw, a_pv, a_tm, a_comp, a_status, _ptr(counts, _lp),
-                               ctypes.byref(mx), ctypes.byref(t))
+        rc = getattr(L, "icikt_pair_list" + sfx)(*lead, gp, ng, _ptr(pi, _ip), _ptr(pj, _ip), P,
+                                                 ctypes.byref(o), a_raw, a_pv, a_tm, a_comp, a_status,
+                                                 _ptr(counts, _lp), ctypes.byref(mx), ctypes.byref(t))
     check(rc)
     out = dict(raw=raw, pvalue=pv, taumax=tm, completeness=comp, status=status,
                max_taumax=mx.value, timings=t.as_dict())
@@ -257,12 +317,10 @@ def run_matrices(data, global_na=(), scale_max=True, diag_good=True, n_good=None
     (scale_and_reshape, R/kendalltau.R:357-421).  Returns the requested matrices plus
     status_counts (pairs per status class), max_taumax and timings.
     devices: list of CUDA ordinals -> icikt_matrices_multi (all pairs only): the pair order is sliced
-    over the devices and every device returns its own block of columns of each matrix."""
+    over the devices and every device returns its own block of columns of each matrix.
+    data may be a scipy.sparse matrix (-> the *_csc entry points)."""
     L = load()
-    data = np.asfortranarray(data, dtype=np.float64)
-    if data.ndim != 2:
-        raise ValueError("data must be a 2-D array (features x samples)")
-    n, C = data.shape
+    lead, sfx, n, C, keep_alive = _matrix_args(data)
     o = make_opts(**opt_kw)
     mats = {k: (np.empty((C, C), dtype=np.float64, order="F") if k in want else None) for k in MATRIX_NAMES}
     hist = np.zeros(NSTATUS, dtype=np.int64)
@@ -277,14 +335,14 @@ def run_matrices(data, global_na=(), scale_max=True, diag_good=True, n_good=None
         if pi is not None:
             raise ValueError("several devices: all pairs only")
         dev = np.ascontiguousarray(list(devices), dtype=np.int32)
-        check(L.icikt_matrices_multi(_ptr(data, _dp), n, C, n, gp, ng, ctypes.byref(o), _ptr(dev, _ip), int(dev.size),
+        check(getattr(L, "icikt_matrices_multi" + sfx)(*lead, gp, ng, ctypes.byref(o), _ptr(dev, _ip), int(dev.size),
                                      int(bool(scale_max)), int(bool(diag_good)), _ptr(ngood, _ip),
                                      *(_ptr(mats[k], _dp) for k in MATRIX_NAMES), _ptr(hist, _lp), ctypes.byref(mx),
                                      ctypes.byref(t)))
         out = {k: v for k, v in mats.items() if v is not None}
         out.update(status_counts=hist, max_taumax=mx.value, timings=t.as_dict())
         return out
-    check(L.icikt_matrices(_ptr(data, _dp), n, C, n, gp, ng, _ptr(pi, _ip), _ptr(pj, _ip),
+    check(getattr(L, "icikt_matrices" + sfx)(*lead, gp, ng, _ptr(pi, _ip), _ptr(pj, _ip),
                            0 if pi is None else int(pi.size), ctypes.byref(o), int(bool(scale_max)),
                            int(bool(diag_good)), _ptr(ngood, _ip), *(_ptr(mats[k], _dp) for k in MATRIX_NAMES),
                            _ptr(hist, _lp), ctypes.byref(mx), ctypes.byref(t)))
@@ -295,10 +353,10 @@ def run_matrices(data, global_na=(), scale_max=True, diag_good=True, n_good=None
 
 def pairwise_completeness(data, global_na=(), pi=None, pj=None, want_matrix=False, want_pairs=True, device=0):
     """icikt_pairwise_completeness: rows missing in either column and 1 - missing/n per pair
-    (all pairs in combn order followed by the diagonal when pi is None)."""
+    (all pairs in combn order followed by the diagonal when pi is None).  data may be a scipy.sparse
+    matrix (-> icikt_pairwise_completeness_csc)."""
     L = load()
-    data = np.asfortranarray(data, dtype=np.float64)
-    n, C = data.shape
+    lead, sfx, n, C, keep_alive = _matrix_args(data)
     if pi is not None:
         pi = np.ascontiguousarray(pi, dtype=np.int32)
         pj = np.ascontiguousarray(pj, dtype=np.int32)
@@ -309,8 +367,8 @@ def pairwise_completeness(data, global_na=(), pi=None, pj=None, want_matrix=Fals
     comp = np.empty(P, dtype=np.float64) if want_pairs else None
     mat = np.empty((C, C), dtype=np.float64, order="F") if want_matrix else None
     g, gp, ng = _global_na_array(global_na)
-    check(L.icikt_pairwise_completeness(_ptr(data, _dp), n, C, n, gp, ng, int(device), _ptr(pi, _ip), _ptr(pj, _ip),
-                                        P, _ptr(missing, _ip), _ptr(comp, _dp), _ptr(mat, _dp)))
+    check(getattr(L, "icikt_pairwise_completeness" + sfx)(*lead, gp, ng, int(device), _ptr(pi, _ip), _ptr(pj, _ip),
+                                                        P, _ptr(missing, _ip), _ptr(comp, _dp), _ptr(mat, _dp)))
     out = dict(missing=missing, completeness=comp) if want_pairs else {}
     if want_matrix:
         out["matrix"] = mat

@@ -71,6 +71,17 @@ def _colnames_of(x, colnames, arg):
             x = x.to_numpy()
     except ImportError:  # pandas is optional
         pass
+    if _lib.is_sparse(x):  # stays sparse: the library takes the stored entries (entries not stored are 0.0)
+        if len(x.shape) != 2:
+            raise ValueError(f"`{arg}` must be matrix-like (features x samples)")
+        if names is None:
+            raise ValueError(f"Colnames of `{arg}` must be be specified.")
+        names = list(names)
+        if len(names) != x.shape[1]:
+            raise ValueError(f"`colnames` has {len(names)} entries but `{arg}` has {x.shape[1]} columns")
+        if not (np.issubdtype(x.dtype, np.floating) or np.issubdtype(x.dtype, np.integer)):
+            raise TypeError(f"`{arg}` must be a numeric type.")
+        return _lib.canonical_csc(x), names
     arr = np.asarray(x)
     if arr.ndim != 2:
         raise ValueError(f"`{arg}` must be matrix-like (features x samples)")
@@ -97,6 +108,27 @@ def setup_missing_matrix(data_matrix, global_na):
         if np.isfinite(v):
             excl |= (data == v)
     return excl
+
+
+def _keep_and_n_good(data, global_na):
+    """keep (C x n: not missing) and n_good (per column) of setup_missing_matrix (R/utils.R:1-23).  For
+    sparse input both come from the stored entries: an entry not stored is 0.0, missing iff global_na holds a 0
+    (the same rule setup_missing_matrix applies to it)."""
+    if not _lib.is_sparse(data):
+        exclude_loc = setup_missing_matrix(data, global_na)
+        return (~exclude_loc).T, (~exclude_loc).sum(axis=0)
+    m = _lib.CSC(data)
+    n, C = m.shape
+    implicit_good = not setup_missing_matrix(np.zeros(1), global_na)[0]
+    stored_good = ~setup_missing_matrix(m.values, global_na)
+    per_col = np.diff(m.colptr)
+    col = np.repeat(np.arange(C), per_col)
+    n_good = np.bincount(col, weights=stored_good, minlength=C).astype(np.int64)
+    if implicit_good:
+        n_good += n - per_col
+    keep = np.full((C, n), implicit_good, dtype=bool)
+    keep[col, m.rowidx] = stored_good
+    return keep, n_good
 
 
 def setup_comparisons(samples, include_only=None, diag_good=True, include_arg="include_only"):
@@ -207,7 +239,7 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     n, C = data.shape
     log.info("Processing missing values ...")
     global_na = [float(v) for v in global_na]
-    exclude_loc = setup_missing_matrix(data, global_na)
+    keep, n_good = _keep_and_n_good(data, global_na)
     log.info("Figuring out comparisons to do ...")
     if include_only is None and return_matrix and not check_timing:
         # every pair, in the library's own order, straight into matrices: no pair list on the host
@@ -238,7 +270,6 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     t1 = time.perf_counter()
     if return_matrix and (n_gpus <= 1 or all_pairs):
         # scale_and_reshape on the device: the five C x C matrices come back filled (:357-421)
-        n_good = (~exclude_loc).sum(axis=0)
         if all_pairs and n_gpus > 1:  # every GPU fills and returns its own block of columns
             r = _lib.run_matrices(data, global_na, scale_max, diag_good, n_good, devices=range(n_gpus), **kw)
         elif all_pairs:
@@ -249,7 +280,7 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
         _warn_status_counts(r["status_counts"])
         log.info("Generating the output matrix ...")
         out = {k: r[k] for k in _lib.MATRIX_NAMES}
-        out["keep"] = (~exclude_loc).T
+        out["keep"] = keep
         out["run_time"] = run_time
         out["names"] = names
         return out
@@ -268,7 +299,6 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
         cor = raw / r["max_taumax"]
     else:
         cor = raw.copy()
-    n_good = (~exclude_loc).sum(axis=0)
     if diag_good:  # R/kendalltau.R:374-386 (appended after scaling, never scaled)
         d = np.arange(C, dtype=np.int32)
         dg = n_good / n_good.max()
@@ -284,7 +314,7 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     log.info("Generating the output matrix ...")
     out = _reshape(names, pi, pj, dict(cor=cor, raw=raw, pvalue=pvalue, taumax=taumax,
                                         completeness=completeness))
-    out["keep"] = (~exclude_loc).T
+    out["keep"] = keep
     out["run_time"] = run_time
     out["names"] = names
     return out

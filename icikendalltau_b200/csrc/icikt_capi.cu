@@ -185,6 +185,13 @@ struct icikt_plan {
   const double* d_data = nullptr;
   int64_t ld = 0;
   double* d_global_na = nullptr;
+  // CSC input (the *_csc entry points): the stored entries on the device, each at its global entry number;
+  // csc_expand_kernel rebuilds d_data_own from them ahead of K1.  Kept with the plan, grown on demand.
+  int64_t* d_colptr = nullptr;  // [C + 1]
+  int32_t* d_rowidx = nullptr;
+  double* d_values = nullptr;
+  int64_t csc_cap = 0;                   // entries d_rowidx / d_values hold
+  int64_t expand_lo = 0, expand_hi = 0;  // columns uploaded as CSC and not expanded yet
 
   ColumnTables tab;
   ColumnWork wk;
@@ -245,8 +252,15 @@ namespace {
 void free_plan(icikt_plan* p) {
   if (!p) return;
   cudaSetDevice(p->device);
+  // a failed call may leave copies in flight: none may still read a caller's array once the call returns
+  if (p->copy_stream) cudaStreamSynchronize(p->copy_stream);
+  if (p->stream) cudaStreamSynchronize(p->stream);
+  cudaGetLastError();
   cudaFree(p->d_data_own);
   cudaFree(p->d_global_na);
+  cudaFree(p->d_colptr);
+  cudaFree(p->d_rowidx);
+  cudaFree(p->d_values);
   cudaFree(p->tab.perm);
   cudaFree(p->tab.rank);
   cudaFree(p->tab.trow);
@@ -372,12 +386,17 @@ int select_device(int device) {
 // memcpy into the caller's (usually freshly allocated, not yet faulted-in) array: one thread moves
 // about 5 GB/s there, a PCIe 5 link delivers ten times that, so large blocks are split over a few
 // threads (ICIKT_COPY_THREADS, default min(8, hardware threads); 1 = plain memcpy)
-void host_copy(void* dst, const void* src, size_t bytes) {
+int copy_threads() {
   static const int n_threads = [] {
     const char* e = std::getenv("ICIKT_COPY_THREADS");
     int t = e ? std::atoi(e) : (int)std::min(8u, std::max(1u, std::thread::hardware_concurrency()));
     return std::max(1, std::min(t, 64));
   }();
+  return n_threads;
+}
+
+void host_copy(void* dst, const void* src, size_t bytes) {
+  const int n_threads = copy_threads();
   constexpr size_t kMinPart = 2u << 20;
   const int parts = (int)std::min<size_t>((size_t)n_threads, bytes / kMinPart);
   if (parts <= 1) {
@@ -470,9 +489,141 @@ bool host_is_pinned(const void* ptr) {
   return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
 }
 
-// host -> device copy of columns [c_lo, c_hi) into the plan's own matrix buffer, on `stream`
-int copy_columns_in(icikt_plan* p, const double* data, int64_t ld, int64_t c_lo, int64_t c_hi, cudaStream_t stream) {
+// Where the columns of a call come from: a dense column-major matrix (data, ld) or a CSC matrix (colptr
+// [C + 1], rowidx / values [colptr[C]], checked by check_csc).
+struct ColumnSource {
+  const double* data = nullptr;
+  int64_t ld = 0;
+  const int64_t* colptr = nullptr;
+  const int32_t* rowidx = nullptr;
+  const double* values = nullptr;
+  bool csc() const { return colptr != nullptr; }
+};
+ColumnSource dense_source(const double* data, int64_t ld) {
+  ColumnSource s;
+  s.data = data;
+  s.ld = ld;
+  return s;
+}
+ColumnSource csc_source(const int64_t* colptr, const int32_t* rowidx, const double* values) {
+  ColumnSource s;
+  s.colptr = colptr;
+  s.rowidx = rowidx;
+  s.values = values;
+  return s;
+}
+
+// first column of [c_lo, c_hi) with a row outside [0, n) or rows that do not strictly increase; c_hi if none
+int64_t first_bad_column(const int64_t* colptr, const int32_t* rowidx, int64_t n, int64_t c_lo, int64_t c_hi) {
+  for (int64_t c = c_lo; c < c_hi; ++c) {
+    int64_t prev = -1;
+    for (int64_t k = colptr[c]; k < colptr[c + 1]; ++k) {
+      const int64_t r = rowidx[k];
+      if (r < 0 || r >= n || r <= prev) return c;
+      prev = r;
+    }
+  }
+  return c_hi;
+}
+
+// The host-side checks of a CSC matrix, before any device work: colptr starts at 0 and never decreases, the
+// arrays exist if there are entries, and the rows of every column lie in [0, n) and strictly increase.  The
+// row scan of a large matrix is split over a few host threads (ICIKT_COPY_THREADS, as the copies); the
+// message names the first bad column either way.
+int check_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C) {
+  if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
+  if (!colptr) return fail(ICIKT_ERR_BAD_ARG, "CSC input: colptr is NULL");
+  if (colptr[0] != 0) return fail(ICIKT_ERR_BAD_ARG, "CSC input: colptr[0] is " + std::to_string(colptr[0]) + ", not 0");
+  for (int64_t c = 0; c < C; ++c)
+    if (colptr[c + 1] < colptr[c])
+      return fail(ICIKT_ERR_BAD_ARG, "CSC input: colptr decreases at column " + std::to_string(c) + " (" +
+                                         std::to_string(colptr[c]) + " -> " + std::to_string(colptr[c + 1]) + ")");
+  const int64_t nnz = colptr[C];
+  if (nnz > 0 && (!rowidx || !values))
+    return fail(ICIKT_ERR_BAD_ARG, "CSC input: colptr[C] = " + std::to_string(nnz) +
+                                       " entries but rowidx or values is NULL");
+  const int parts = (int)std::min<int64_t>(std::min<int64_t>(copy_threads(), C), nnz >> 20);
+  int64_t bad = C;
+  if (parts <= 1) {
+    bad = first_bad_column(colptr, rowidx, n, 0, C);
+  } else {  // column ranges of about equal entry counts
+    std::vector<int64_t> lo((size_t)parts + 1, C), found((size_t)parts, C);
+    lo[0] = 0;
+    for (int t = 1; t < parts; ++t)
+      lo[(size_t)t] = std::upper_bound(colptr, colptr + C + 1, nnz * t / parts) - colptr - 1;
+    std::vector<std::thread> th;
+    for (int t = 1; t < parts; ++t)
+      th.emplace_back([&, t] { found[(size_t)t] = first_bad_column(colptr, rowidx, n, lo[(size_t)t], lo[(size_t)t + 1]); });
+    found[0] = first_bad_column(colptr, rowidx, n, 0, lo[1]);
+    for (auto& x : th) x.join();
+    for (int t = 0; t < parts; ++t)
+      if (found[(size_t)t] < lo[(size_t)t + 1]) { bad = found[(size_t)t]; break; }
+  }
+  if (bad == C) return ICIKT_OK;
+  int64_t prev = -1;
+  for (int64_t k = colptr[bad];; ++k) {  // first_bad_column stopped inside this column
+    const int64_t r = rowidx[k];
+    if (r < 0 || r >= n)
+      return fail(ICIKT_ERR_BAD_ARG, "CSC input: row " + std::to_string(r) + " of column " + std::to_string(bad) +
+                                         " is outside [0, " + std::to_string(n) + ")");
+    if (r <= prev)
+      return fail(ICIKT_ERR_BAD_ARG, "CSC input: rows of column " + std::to_string(bad) +
+                                         (r == prev ? " repeat row " + std::to_string(r)
+                                                    : " are not sorted (" + std::to_string(prev) + " before " +
+                                                          std::to_string(r) + ")"));
+    prev = r;
+  }
+}
+
+// host -> device copy of a contiguous array; pageable memory of 8 MB and more goes through the plan's pinned
+// chunks (staged_copy_in), as a dense matrix does
+int copy_array_in(icikt_plan* p, void* d_dst, const void* src, size_t bytes, cudaStream_t stream) {
+  if (bytes == 0) return ICIKT_OK;
+  if (bytes >= (8u << 20) && !std::getenv("ICIKT_NO_STAGED_UPLOAD") && !host_is_pinned(src))
+    return staged_copy_in(p, d_dst, src, bytes, stream);
+  CK(cudaMemcpyAsync(d_dst, src, bytes, cudaMemcpyHostToDevice, stream));
+  return ICIKT_OK;
+}
+
+// CSC columns [c_lo, c_hi): the colptr slice and the slices [colptr[c_lo], colptr[c_hi]) of rowidx and values,
+// on `stream`.  The columns are expanded into d_data_own by the next plan_columns_impl, on the compute stream.
+// (Neighbouring chunks of a pipelined call both copy their shared colptr entry; the second copy writes the
+// value the expansion of the first chunk may be reading.)
+int copy_csc_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, cudaStream_t stream) {
+  const int64_t nnz = s.colptr[p->C];
+  if (!p->d_colptr) CK(dmalloc(&p->d_colptr, (size_t)p->C + 1));
+  if (nnz > p->csc_cap) {  // nothing of an earlier call is in flight: every call ends with its streams idle
+    cudaFree(p->d_rowidx);
+    cudaFree(p->d_values);
+    p->d_rowidx = nullptr;
+    p->d_values = nullptr;
+    p->csc_cap = 0;
+    CK(dmalloc(&p->d_rowidx, (size_t)nnz));
+    CK(dmalloc(&p->d_values, (size_t)nnz));
+    p->csc_cap = nnz;
+  }
+  p->expand_lo = p->expand_hi = 0;
+  if (c_hi <= c_lo) return ICIKT_OK;
+  const int64_t k_lo = s.colptr[c_lo], k_hi = s.colptr[c_hi];
+  CK(cudaMemcpyAsync(p->d_colptr + c_lo, s.colptr + c_lo, sizeof(int64_t) * (size_t)(c_hi - c_lo + 1),
+                     cudaMemcpyHostToDevice, stream));
+  int rc = copy_array_in(p, p->d_rowidx + k_lo, s.rowidx + k_lo, sizeof(int32_t) * (size_t)(k_hi - k_lo), stream);
+  if (rc == ICIKT_OK)
+    rc = copy_array_in(p, p->d_values + k_lo, s.values + k_lo, sizeof(double) * (size_t)(k_hi - k_lo), stream);
+  if (rc != ICIKT_OK) return rc;
+  p->expand_lo = c_lo;
+  p->expand_hi = c_hi;
+  return ICIKT_OK;
+}
+
+// host -> device copy of columns [c_lo, c_hi) into the plan's own matrix buffer (CSC: of their stored
+// entries), on `stream`
+int copy_columns_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, cudaStream_t stream) {
   if (!p->d_data_own) CK(dmalloc(&p->d_data_own, (size_t)p->n * p->C));
+  if (s.csc()) return copy_csc_in(p, s, c_lo, c_hi, stream);
+  p->expand_lo = p->expand_hi = 0;
+  const double* data = s.data;
+  const int64_t ld = s.ld;
   if (c_hi <= c_lo) return ICIKT_OK;
   const size_t bytes = sizeof(double) * (size_t)p->n * (size_t)(c_hi - c_lo);
   if (ld == p->n && bytes >= (8u << 20) && !std::getenv("ICIKT_NO_STAGED_UPLOAD") && !host_is_pinned(data + (size_t)c_lo * ld))
@@ -482,10 +633,10 @@ int copy_columns_in(icikt_plan* p, const double* data, int64_t ld, int64_t c_lo,
   return ICIKT_OK;
 }
 
-int upload_columns(icikt_plan* p, const double* data, int64_t ld, int64_t c_lo, int64_t c_hi) {
+int upload_columns(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi) {
   CK(cudaSetDevice(p->device));
   CK(cudaEventRecord(p->ev[0], p->stream));
-  const int rc = copy_columns_in(p, data, ld, c_lo, c_hi, p->stream);
+  const int rc = copy_columns_in(p, s, c_lo, c_hi, p->stream);
   if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[1], p->stream));
   p->d_data = p->d_data_own;
@@ -697,13 +848,14 @@ int64_t icikt_plan_num_pairs(const icikt_plan* p) { return p ? p->P : 0; }
 
 int icikt_plan_upload(icikt_plan* p, const double* data, int64_t ld) {
   if (!p || !data || ld < p->n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
-  return upload_columns(p, data, ld, 0, p->C);
+  return upload_columns(p, dense_source(data, ld), 0, p->C);
 }
 
 int icikt_plan_set_device_matrix(icikt_plan* p, const double* d_data, int64_t ld) {
   if (!p || !d_data || ld < p->n) return fail(ICIKT_ERR_BAD_ARG, "bad device matrix arguments");
   p->d_data = d_data;
   p->ld = ld;
+  p->expand_lo = p->expand_hi = 0;
   p->columns_done = false;
   p->pairs_done = false;
   CK(cudaSetDevice(p->device));
@@ -736,6 +888,14 @@ static int plan_columns_impl(icikt_plan* p, const double* global_na, int32_t n_g
   if (nlit) CK(cudaMemcpyAsync(p->d_global_na, lit, sizeof(double) * nlit, cudaMemcpyHostToDevice, p->stream));
   if (reset) CK(cudaMemsetAsync(p->tab.max_tied, 0, 4 * sizeof(int32_t), p->stream));
   CK(cudaEventRecord(e0 ? e0 : p->ev[2], p->stream));
+  // columns uploaded as CSC become dense first (their copies precede this point on the stream)
+  int expand_launches = 0;
+  if (p->expand_hi > p->expand_lo) {
+    expand_launches = launch_csc_expand(p->d_colptr, p->d_rowidx, p->d_values, p->n, p->expand_lo, p->expand_hi,
+                                        p->d_data_own, p->stream);
+    if (expand_launches < 0) return launch_fail("CSC expansion kernel");
+    p->expand_lo = p->expand_hi = 0;
+  }
   // the largest tier decides whether the global scratch may be needed at all
   const int64_t n_units = (int64_t)p->units.size();
   const bool inplace_ok = p->opts.perspective != ICIKT_PERSPECTIVE_COMPLETE;  // that mode has no in-place kernel
@@ -762,9 +922,10 @@ static int plan_columns_impl(icikt_plan* p, const double* global_na, int32_t n_g
     sh->scratch_stride = p->d_scratch ? slot_bytes : 0;
     sh->scratch_ctas = p->d_scratch ? (int)std::min<size_t>((size_t)slot_ctas, p->scratch_bytes / (size_t)slot_bytes) : 0;
   }
-  const int l = launch_columns(p->d_data, p->ld, p->d_global_na, nlit, na_inf, p->tab, p->wk, p->shape,
-                               p->d_scratch, p->stream, col_lo, col_hi);
-  if (l < 0) return launch_fail("column kernels");
+  const int lc = launch_columns(p->d_data, p->ld, p->d_global_na, nlit, na_inf, p->tab, p->wk, p->shape,
+                                p->d_scratch, p->stream, col_lo, col_hi);
+  if (lc < 0) return launch_fail("column kernels");
+  const int l = lc + expand_launches;
   CK(cudaEventRecord(e1 ? e1 : p->ev[3], p->stream));
   // no synchronisation: `lit` is pageable host memory, so the copy above was staged before
   // cudaMemcpyAsync returned
@@ -799,7 +960,7 @@ int icikt_plan_columns_finish(icikt_plan* p) {
 int icikt_plan_upload_columns(icikt_plan* p, const double* data, int64_t ld, int64_t col_lo, int64_t col_hi) {
   if (!p || !data || ld < p->n || col_lo < 0 || col_hi > p->C || col_lo > col_hi)
     return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
-  return upload_columns(p, data, ld, col_lo, col_hi);
+  return upload_columns(p, dense_source(data, ld), col_lo, col_hi);
 }
 
 int icikt_plan_tables(icikt_plan* p, icikt_table* out, int32_t cap) {
@@ -1105,11 +1266,11 @@ void icikt_plan_destroy(icikt_plan* p) { free_plan(p); }
 // a finished row block back on the copy stream while the next block runs.  `download` false: the results
 // stay on the device (matrix output follows).  Same results as upload + columns + pairs + download: only
 // the order in which the pairs are computed differs.
-static int run_staged(icikt_plan* p, const double* data, int64_t ld, const double* global_na, int32_t n_global_na,
+static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
                       bool download, double* raw, double* pvalue, double* taumax, double* completeness,
                       int32_t* status, int64_t* counts, double* max_taumax) {
   if (!p || !p->staged) return fail(ICIKT_ERR_BAD_ARG, "not a staged plan");
-  if (!data || ld < p->n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
+  if (!s.csc() && (!s.data || s.ld < p->n)) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
   if (counts && !p->d_counts) return fail(ICIKT_ERR_BAD_ARG, "plan was created without want_counts");
   CK(cudaSetDevice(p->device));
   if (!p->d_data_own) CK(dmalloc(&p->d_data_own, (size_t)p->n * p->C));
@@ -1127,7 +1288,7 @@ static int run_staged(icikt_plan* p, const double* data, int64_t ld, const doubl
     const StageLaunch& st = p->stages[l];
     cudaEvent_t* te = &p->time_ev[5 * l];
     if (st.col_hi > st.col_lo) {
-      int rc = copy_columns_in(p, data, ld, st.col_lo, st.col_hi, p->copy_stream);
+      int rc = copy_columns_in(p, s, st.col_lo, st.col_hi, p->copy_stream);
       if (rc != ICIKT_OK) return rc;
       CK(cudaEventRecord(p->sync_ev[2 * l], p->copy_stream));
       if (st.col_hi == p->C) CK(cudaEventRecord(p->ev[1], p->copy_stream));
@@ -1240,12 +1401,12 @@ struct MatrixOut {  // the download step of one_shot as matrices instead of per-
   int64_t* status_counts;
 };
 
-static int one_shot(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+static int one_shot(const ColumnSource& s, int64_t n, int64_t C, const double* global_na,
                     int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
                     const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
                     double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
                     icikt_timings* timings, const MatrixOut* mat = nullptr) {
-  if (!data || (!raw && !mat)) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
+  if ((!s.data && !s.csc()) || (!raw && !mat)) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
   icikt_opts o;
   if (opts) o = *opts; else icikt_default_opts(&o);
   o.want_counts = counts ? 1 : 0;
@@ -1269,10 +1430,10 @@ static int one_shot(const double* data, int64_t n, int64_t C, int64_t ld, const 
     if (cacheable) g_cached = p;
   }
   if (staged) {
-    rc = run_staged(p, data, ld, global_na, n_global_na, mat == nullptr, raw, pvalue, taumax, completeness, status,
+    rc = run_staged(p, s, global_na, n_global_na, mat == nullptr, raw, pvalue, taumax, completeness, status,
                     counts, max_taumax);
   } else {
-    rc = icikt_plan_upload(p, data, ld);
+    rc = s.csc() ? upload_columns(p, s, 0, C) : icikt_plan_upload(p, s.data, s.ld);
     if (rc == ICIKT_OK) rc = icikt_plan_columns(p, global_na, n_global_na);
     if (rc == ICIKT_OK) rc = icikt_plan_pairs(p);
   }
@@ -1380,15 +1541,27 @@ int icikt_all_pairs(const double* data, int64_t n, int64_t C, int64_t ld, const 
                     int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue,
                     double* taumax, double* completeness, int32_t* status, int64_t* counts,
                     double* max_taumax, icikt_timings* timings) {
-  return one_shot(data, n, C, ld, global_na, n_global_na, nullptr, nullptr, 0, opts, raw, pvalue, taumax,
-                  completeness, status, counts, max_taumax, timings);
+  return one_shot(dense_source(data, ld), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw, pvalue,
+                  taumax, completeness, status, counts, max_taumax, timings);
 }
 
-int icikt_matrices(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                   int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts* opts,
-                   int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
-                   double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
-                   double* max_taumax, icikt_timings* timings) {
+int icikt_all_pairs_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                        const double* global_na, int32_t n_global_na, const icikt_opts* opts, double* raw,
+                        double* pvalue, double* taumax, double* completeness, int32_t* status, int64_t* counts,
+                        double* max_taumax, icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return one_shot(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw,
+                  pvalue, taumax, completeness, status, counts, max_taumax, timings);
+}
+
+}  // extern "C"
+
+static int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                         const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts* opts, int32_t scale_max,
+                         int32_t diag_good, const int32_t* n_good, double* cor, double* raw, double* pvalue,
+                         double* taumax, double* completeness, int64_t* status_counts, double* max_taumax,
+                         icikt_timings* timings) {
   if ((pi == nullptr) != (pj == nullptr)) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must both be given");
   icikt_opts o;
   if (opts) o = *opts; else icikt_default_opts(&o);
@@ -1396,14 +1569,38 @@ int icikt_matrices(const double* data, int64_t n, int64_t C, int64_t ld, const d
     return fail(ICIKT_ERR_BAD_ARG, "matrix output needs the whole pair order on one device");
   if (!pi) o.include_diag = diag_good ? 0 : 1;  // setup_comparisons, R/kendalltau.R:191-194
   const MatrixOut mo{scale_max, diag_good, n_good, cor, status_counts};
-  return one_shot(data, n, C, ld, global_na, n_global_na, pi, pj, P, &o, raw, pvalue, taumax, completeness,
-                  nullptr, nullptr, max_taumax, timings, &mo);
+  return one_shot(s, n, C, global_na, n_global_na, pi, pj, P, &o, raw, pvalue, taumax, completeness, nullptr, nullptr,
+                  max_taumax, timings, &mo);
 }
 
-int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                                int32_t n_global_na, int32_t device, const int32_t* pi, const int32_t* pj,
-                                int64_t P, int32_t* missing, double* completeness, double* matrix) {
-  if (!data || n < 1 || C < 1 || ld < n) return fail(ICIKT_ERR_BAD_ARG, "bad matrix arguments");
+extern "C" {
+
+int icikt_matrices(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                   int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts* opts,
+                   int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
+                   double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
+                   double* max_taumax, icikt_timings* timings) {
+  return matrices_impl(dense_source(data, ld), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max, diag_good,
+                       n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
+}
+
+int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                       const double* global_na, int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
+                       const icikt_opts* opts, int32_t scale_max, int32_t diag_good, const int32_t* n_good,
+                       double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                       int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return matrices_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max,
+                       diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
+}
+
+}  // extern "C"
+
+static int pairwise_completeness_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na,
+                                      int32_t n_global_na, int32_t device, const int32_t* pi, const int32_t* pj,
+                                      int64_t P, int32_t* missing, double* completeness, double* matrix) {
+  if ((!s.csc() && (!s.data || s.ld < n)) || n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "bad matrix arguments");
   if ((pi == nullptr) != (pj == nullptr)) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must both be given");
   if (n_global_na < 0 || (n_global_na > 0 && !global_na)) return fail(ICIKT_ERR_BAD_ARG, "bad global_na");
   if (matrix && pi) return fail(ICIKT_ERR_BAD_ARG, "the matrix output covers all pairs; pass pi = pj = NULL");
@@ -1426,13 +1623,16 @@ int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_
   const int64_t words = (n + 31) / 32;
   const bool per_pair = missing || completeness;
   struct Buffers {
-    double *data = nullptr, *lit = nullptr, *comp = nullptr, *mat = nullptr;
+    double *data = nullptr, *lit = nullptr, *comp = nullptr, *mat = nullptr, *values = nullptr;
     uint32_t* bits = nullptr;
-    int32_t *pi = nullptr, *pj = nullptr, *miss = nullptr;
+    int32_t *pi = nullptr, *pj = nullptr, *miss = nullptr, *rowidx = nullptr;
+    int64_t* colptr = nullptr;
     cudaStream_t stream = nullptr;
     ~Buffers() {
+      if (stream) cudaStreamSynchronize(stream);  // no copy still reads the caller's arrays after an error
       cudaFree(data); cudaFree(lit); cudaFree(comp); cudaFree(mat); cudaFree(bits);
       cudaFree(pi); cudaFree(pj); cudaFree(miss);
+      cudaFree(colptr); cudaFree(rowidx); cudaFree(values);
       if (stream) cudaStreamDestroy(stream);
     }
   } b;
@@ -1440,8 +1640,22 @@ int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_
   CK(dmalloc(&b.data, (size_t)n * C));
   CK(dmalloc(&b.lit, 64));
   CK(dmalloc(&b.bits, (size_t)words * C));
-  CK(cudaMemcpy2DAsync(b.data, sizeof(double) * n, data, sizeof(double) * ld, sizeof(double) * n, (size_t)C,
-                       cudaMemcpyHostToDevice, b.stream));
+  if (s.csc()) {  // the stored entries, expanded into the dense matrix on the device
+    const int64_t nnz = s.colptr[C];
+    CK(dmalloc(&b.colptr, (size_t)C + 1));
+    CK(dmalloc(&b.rowidx, (size_t)nnz));
+    CK(dmalloc(&b.values, (size_t)nnz));
+    CK(cudaMemcpyAsync(b.colptr, s.colptr, sizeof(int64_t) * (size_t)(C + 1), cudaMemcpyHostToDevice, b.stream));
+    if (nnz) {
+      CK(cudaMemcpyAsync(b.rowidx, s.rowidx, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, b.stream));
+      CK(cudaMemcpyAsync(b.values, s.values, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, b.stream));
+    }
+    if (launch_csc_expand(b.colptr, b.rowidx, b.values, n, 0, C, b.data, b.stream) < 0)
+      return launch_fail("CSC expansion kernel");
+  } else {
+    CK(cudaMemcpy2DAsync(b.data, sizeof(double) * n, s.data, sizeof(double) * s.ld, sizeof(double) * n, (size_t)C,
+                         cudaMemcpyHostToDevice, b.stream));
+  }
   if (nlit) CK(cudaMemcpyAsync(b.lit, lit, sizeof(double) * nlit, cudaMemcpyHostToDevice, b.stream));
   if (launch_missing_bits(b.data, n, n, C, b.lit, nlit, na_nan, na_inf, b.bits, words, b.stream) < 0)
     return launch_fail("missing-mask kernel");
@@ -1469,6 +1683,25 @@ int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_
   return ICIKT_OK;
 }
 
+extern "C" {
+
+int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                                int32_t n_global_na, int32_t device, const int32_t* pi, const int32_t* pj,
+                                int64_t P, int32_t* missing, double* completeness, double* matrix) {
+  return pairwise_completeness_impl(dense_source(data, ld), n, C, global_na, n_global_na, device, pi, pj, P, missing,
+                                    completeness, matrix);
+}
+
+int icikt_pairwise_completeness_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                                    int64_t C, const double* global_na, int32_t n_global_na, int32_t device,
+                                    const int32_t* pi, const int32_t* pj, int64_t P, int32_t* missing,
+                                    double* completeness, double* matrix) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return pairwise_completeness_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, device, pi, pj,
+                                    P, missing, completeness, matrix);
+}
+
 }  // extern "C"
 
 namespace {
@@ -1480,8 +1713,8 @@ namespace {
 // copies: K1 is not replicated and the raw matrix never travels between devices); otherwise every
 // device uploads the whole matrix and preprocesses all columns.
 struct MultiJob {
-  const double* data;
-  int64_t n, C, ld;
+  ColumnSource src;
+  int64_t n, C;
   const double* global_na;
   int32_t n_global_na;
   icikt_opts base;
@@ -1551,10 +1784,10 @@ int multi_worker_pairs(MultiJob& J, int k, icikt_plan** out) {
   *out = p;
   if (!J.gather) {
     if (cnt <= 0) return rc;
-    if (rc == ICIKT_OK) rc = icikt_plan_upload(p, J.data, J.ld);
+    if (rc == ICIKT_OK) rc = J.src.csc() ? upload_columns(p, J.src, 0, J.C) : icikt_plan_upload(p, J.src.data, J.src.ld);
     if (rc == ICIKT_OK) rc = icikt_plan_columns(p, J.global_na, J.n_global_na);
   } else {
-    if (rc == ICIKT_OK) rc = upload_columns(p, J.data, J.ld, J.col_lo(k), J.col_lo(k + 1));
+    if (rc == ICIKT_OK) rc = upload_columns(p, J.src, J.col_lo(k), J.col_lo(k + 1));
     if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
     if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "column slice");
     J.peer_plan[(size_t)k] = (rc == ICIKT_OK) ? p : nullptr;
@@ -1615,20 +1848,15 @@ int multi_collect(const std::vector<MultiWork>& work, double* max_taumax, icikt_
   return ICIKT_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int icikt_all_pairs_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                          int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
-                          int32_t n_devices, double* raw, double* pvalue, double* taumax,
-                          double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
-                          icikt_timings* timings) {
-  if (!data || !raw) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
+int all_pairs_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                         const icikt_opts* opts, const int32_t* devices, int32_t n_devices, double* raw,
+                         double* pvalue, double* taumax, double* completeness, int32_t* status, int64_t* counts,
+                         double* max_taumax, icikt_timings* timings) {
+  if ((!s.data && !s.csc()) || !raw) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
   if (n_devices < 1 || n_devices > 64) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..64");
   if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
   MultiJob J(n_devices);
-  J.data = data; J.n = n; J.C = C; J.ld = ld; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
   J.devices = devices;
   if (opts) J.base = *opts; else icikt_default_opts(&J.base);
   J.base.want_counts = counts ? 1 : 0;
@@ -1658,12 +1886,12 @@ int icikt_all_pairs_multi(const double* data, int64_t n, int64_t C, int64_t ld, 
   return multi_collect(work, max_taumax, timings);
 }
 
-int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                         int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
-                         int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
-                         double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
-                         double* max_taumax, icikt_timings* timings) {
-  if (!data) return fail(ICIKT_ERR_BAD_ARG, "data must not be NULL");
+int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                        const icikt_opts* opts, const int32_t* devices, int32_t n_devices, int32_t scale_max,
+                        int32_t diag_good, const int32_t* n_good, double* cor, double* raw, double* pvalue,
+                        double* taumax, double* completeness, int64_t* status_counts, double* max_taumax,
+                        icikt_timings* timings) {
+  if (!s.data && !s.csc()) return fail(ICIKT_ERR_BAD_ARG, "data must not be NULL");
   if (n_devices < 1 || n_devices > kMaxMatrixDevices) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..16");
   if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
   icikt_opts base;
@@ -1672,7 +1900,7 @@ int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, c
   base.pair_lo = base.pair_hi = 0;
   const int64_t ptot = tri_pairs(C) + (base.include_diag ? C : 0);
   MultiJob J(n_devices);
-  J.data = data; J.n = n; J.C = C; J.ld = ld; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
   J.devices = devices; J.base = base; J.base.want_counts = 0; J.ptot = ptot;
   {
     std::lock_guard<std::mutex> lock(g_cache_mu);
@@ -1681,8 +1909,8 @@ int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, c
   if (n_devices == 1 || !J.peers_ok || ptot < n_devices || C < n_devices) {
     // one device, or devices that cannot read each other's results: the single-device path
     base.device = J.device_of(0);
-    return icikt_matrices(data, n, C, ld, global_na, n_global_na, nullptr, nullptr, 0, &base, scale_max, diag_good, n_good,
-                          cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
+    return matrices_impl(s, n, C, global_na, n_global_na, nullptr, nullptr, 0, &base, scale_max, diag_good, n_good,
+                         cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
   }
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
   double* outs[5] = {cor, raw, pvalue, taumax, completeness};
@@ -1794,14 +2022,72 @@ int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, c
   return ICIKT_OK;
 }
 
+}  // namespace
+
+extern "C" {
+
+int icikt_all_pairs_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                          int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
+                          int32_t n_devices, double* raw, double* pvalue, double* taumax,
+                          double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
+                          icikt_timings* timings) {
+  return all_pairs_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, raw,
+                              pvalue, taumax, completeness, status, counts, max_taumax, timings);
+}
+
+int icikt_all_pairs_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                              int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                              const int32_t* devices, int32_t n_devices, double* raw, double* pvalue, double* taumax,
+                              double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
+                              icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return all_pairs_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices,
+                              n_devices, raw, pvalue, taumax, completeness, status, counts, max_taumax, timings);
+}
+
+int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                         int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                         int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
+                         double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
+                         double* max_taumax, icikt_timings* timings) {
+  return matrices_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, scale_max,
+                             diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax,
+                             timings);
+}
+
+int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                             const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                             const int32_t* devices, int32_t n_devices, int32_t scale_max, int32_t diag_good,
+                             const int32_t* n_good, double* cor, double* raw, double* pvalue, double* taumax,
+                             double* completeness, int64_t* status_counts, double* max_taumax,
+                             icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return matrices_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices,
+                             n_devices, scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness,
+                             status_counts, max_taumax, timings);
+}
+
 int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
                     int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
                     const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
                     double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
                     icikt_timings* timings) {
   if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
-  return one_shot(data, n, C, ld, global_na, n_global_na, pi, pj, P, opts, raw, pvalue, taumax,
+  return one_shot(dense_source(data, ld), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue, taumax,
                   completeness, status, counts, max_taumax, timings);
+}
+
+int icikt_pair_list_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                        const double* global_na, int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
+                        const icikt_opts* opts, double* raw, double* pvalue, double* taumax, double* completeness,
+                        int32_t* status, int64_t* counts, double* max_taumax, icikt_timings* timings) {
+  if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return one_shot(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue,
+                  taumax, completeness, status, counts, max_taumax, timings);
 }
 
 int icikt_pnorm_device(const double* z, int64_t n, int32_t lower_tail, double* out, int32_t device) {

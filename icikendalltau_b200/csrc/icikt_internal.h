@@ -195,6 +195,12 @@ int launch_pair_missing(const uint32_t* bits, int64_t words, int64_t n, int64_t 
 int launch_missing_matrix(const uint32_t* bits, int64_t words, int64_t n, int64_t C, double* matrix,
                           cudaStream_t stream);
 
+// CSC input (colptr [C + 1], rowidx / values indexed by the global entry number, rows strictly increasing
+// within a column) -> columns [c_lo, c_hi) of the dense column-major n x C matrix `out` (ld = n): stored rows
+// get their value, every other row 0.0
+int launch_csc_expand(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t c_lo,
+                      int64_t c_hi, double* out, cudaStream_t stream);
+
 int launch_pnorm(const double* d_z, int64_t n, int lower, double* d_out, cudaStream_t stream);
 
 int64_t tiled_max_n();

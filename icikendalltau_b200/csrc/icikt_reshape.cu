@@ -1,7 +1,8 @@
 // icikt_reshape.cu -- the result formats either side of the pair kernel, on the device:
 //   * scale_and_reshape (R/kendalltau.R:357-421): per-pair results -> symmetric C x C matrices,
 //     cor = raw / max(taumax), the diagonal of diag_good (:374-386);
-//   * pairwise_completeness (R/kendalltau.R:563-629): missing-row bit masks and popc(x | y).
+//   * pairwise_completeness (R/kendalltau.R:563-629): missing-row bit masks and popc(x | y);
+//   * CSC (sparse) input expanded into the dense column-major matrix the column kernels read.
 // All of it is HBM-bound byte moving; nothing here touches shared memory or tensor cores.
 #include "icikt_internal.h"
 
@@ -148,6 +149,27 @@ __global__ void __launch_bounds__(256) missing_matrix_kernel(const uint32_t* __r
   m[i + j * C] = 1.0 - (double)cnt / (double)n;
 }
 
+// CSC input -> dense columns [c_lo, c_lo + gridDim.x) of `out` (ld = n), one CTA per column: the CTA zero-fills
+// its column with 16-byte stores (a column that starts on an odd element writes that one alone), then, after a
+// barrier, scatters the column's stored entries.  rowidx / values are read coalesced; the rows of a column are
+// sorted, so the scattered writes of a warp mostly fall into a few segments.
+__global__ void __launch_bounds__(512) csc_expand_kernel(const int64_t* __restrict__ colptr,
+                                                         const int32_t* __restrict__ rowidx,
+                                                         const double* __restrict__ values, long long n,
+                                                         long long c_lo, double* __restrict__ out) {
+  const long long c = c_lo + blockIdx.x;
+  double* col = out + c * n;
+  const long long head = (reinterpret_cast<uintptr_t>(col) & 15) ? 1 : 0;
+  const long long pairs = (n - head) >> 1;
+  double2* body = reinterpret_cast<double2*>(col + head);
+  for (long long k = threadIdx.x; k < pairs; k += blockDim.x) body[k] = make_double2(0.0, 0.0);
+  if (threadIdx.x == 0 && head) col[0] = 0.0;
+  if (threadIdx.x == 0 && head + 2 * pairs < n) col[n - 1] = 0.0;
+  __syncthreads();
+  const long long e = colptr[c + 1];
+  for (long long k = colptr[c] + threadIdx.x; k < e; k += blockDim.x) col[rowidx[k]] = values[k];
+}
+
 // Multi-GPU matrix output: this device fills columns [c_lo, c_hi) of the five C x C matrices -- a
 // contiguous block of every (column-major) matrix, so that it leaves for the caller's arrays as one
 // copy per matrix.  The value of entry (r, c) is the result of pair (min, max) wherever that pair was
@@ -248,6 +270,13 @@ int launch_missing_matrix(const uint32_t* bits, int64_t words, int64_t n, int64_
   if (C > 65535) return -1;  // gridDim.y
   const dim3 grid((unsigned)((C + 255) / 256), (unsigned)C);
   missing_matrix_kernel<<<grid, 256, 0, stream>>>(bits, words, n, C, matrix);
+  return launch_status(1);
+}
+
+int launch_csc_expand(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t c_lo,
+                      int64_t c_hi, double* out, cudaStream_t stream) {
+  if (c_hi <= c_lo) return 0;
+  csc_expand_kernel<<<(unsigned)(c_hi - c_lo), 512, 0, stream>>>(colptr, rowidx, values, n, c_lo, out);
   return launch_status(1);
 }
 

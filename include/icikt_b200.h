@@ -103,8 +103,8 @@ typedef struct icikt_opts {
  * pairs_ms and epilogue_ms are then sums over its launches, h2d_ms runs from the start of the call until
  * the last column has landed, d2h_ms from the first result copy to the last, and the parts exceed total_ms. */
 typedef struct icikt_timings { /* milliseconds, CUDA events on the library's streams */
-  float h2d_ms;      /* host -> device copy of the data matrix                        */
-  float columns_ms;  /* per-column preprocessing kernels (K1)                         */
+  float h2d_ms;      /* host -> device copy of the data matrix (CSC input: of its arrays) */
+  float columns_ms;  /* per-column preprocessing kernels (K1; CSC input: with the expansion) */
   float pairs_ms;    /* pair kernel (K2) alone                                        */
   float epilogue_ms; /* fp64 epilogue kernel (K3)                                     */
   float d2h_ms;      /* device -> host copy of the results                            */
@@ -184,6 +184,50 @@ int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_
                                 const double* global_na, int32_t n_global_na, int32_t device,
                                 const int32_t* pi, const int32_t* pj, int64_t P, int32_t* missing,
                                 double* completeness, double* matrix);
+
+/* ---- sparse (CSC) input: the six calls above with (data, n, C, ld) replaced by a compressed sparse
+ * column matrix (colptr, rowidx, values, n, C), the layout of scipy.sparse.csc_matrix, AnnData's X and R's
+ * dgCMatrix: the stored entries of column c are rows rowidx[colptr[c] .. colptr[c+1]) with values[] at the
+ * same positions; colptr has C + 1 entries, colptr[0] = 0, colptr[C] = nnz.  Within a column the rows must
+ * lie in [0, n) and strictly increase (sorted, no duplicates).  An entry that is not stored is the value
+ * 0.0, and every value -- stored or not -- then goes through the usual missing-value rules: with the
+ * default global_na = c(NA, Inf, 0) the stored entries are exactly the present values.  Each result is
+ * bit for bit the dense call's on the expanded matrix.  The arrays are checked on the host before any
+ * device work (ICIKT_ERR_BAD_ARG naming the column).  Only the stored entries travel to the device, where
+ * a kernel rebuilds the dense columns ahead of the per-column preprocessing; in `timings`, h2d_ms covers
+ * the copies of the CSC arrays and columns_ms includes that expansion.                                 */
+int icikt_all_pairs_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                        int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                        double* raw, double* pvalue, double* taumax, double* completeness, int32_t* status,
+                        int64_t* counts, double* max_taumax, icikt_timings* timings);
+int icikt_all_pairs_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                              int64_t C, const double* global_na, int32_t n_global_na,
+                              const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                              double* raw, double* pvalue, double* taumax, double* completeness,
+                              int32_t* status, int64_t* counts, double* max_taumax,
+                              icikt_timings* timings);
+int icikt_pair_list_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                        int64_t C, const double* global_na, int32_t n_global_na, const int32_t* pi,
+                        const int32_t* pj, int64_t P, const icikt_opts* opts, double* raw,
+                        double* pvalue, double* taumax, double* completeness, int32_t* status,
+                        int64_t* counts, double* max_taumax, icikt_timings* timings);
+int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                       int64_t C, const double* global_na, int32_t n_global_na, const int32_t* pi,
+                       const int32_t* pj, int64_t P, const icikt_opts* opts, int32_t scale_max,
+                       int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
+                       double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
+                       double* max_taumax, icikt_timings* timings);
+int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values,
+                             int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                             const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                             int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor,
+                             double* raw, double* pvalue, double* taumax, double* completeness,
+                             int64_t* status_counts, double* max_taumax, icikt_timings* timings);
+int icikt_pairwise_completeness_csc(const int64_t* colptr, const int32_t* rowidx, const double* values,
+                                    int64_t n, int64_t C, const double* global_na,
+                                    int32_t n_global_na, int32_t device, const int32_t* pi,
+                                    const int32_t* pj, int64_t P, int32_t* missing,
+                                    double* completeness, double* matrix);
 
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
