@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("ICIKT_LIB_PATH") or os.path.join(_HERE, "libicikt_b200.so")
 
 OK = 0
-ERR_NO_DEVICE, ERR_BAD_ARG, ERR_TOO_LONG, ERR_CUDA, ERR_ALLOC = -1, -2, -3, -4, -5
+ERR_NO_DEVICE, ERR_BAD_ARG, ERR_TOO_LONG, ERR_CUDA, ERR_ALLOC, ERR_LIMIT = -1, -2, -3, -4, -5, -6
 NCOUNTS = 7
 KERNEL_TILED, KERNEL_NAIVE = 0, 1
 PERSPECTIVE = {"global": 0, "local": 1, "complete": 2}
@@ -35,6 +35,8 @@ EXPORTS = [
     "icikt_matrices_multi", "icikt_stage_table", "icikt_launch_shape",
     "icikt_all_pairs_csc", "icikt_all_pairs_multi_csc", "icikt_pair_list_csc", "icikt_matrices_csc",
     "icikt_matrices_multi_csc", "icikt_pairwise_completeness_csc",
+    "icikt_all_pairs_edges", "icikt_all_pairs_edges_csc", "icikt_edges_count", "icikt_edges_copy",
+    "icikt_edges_free",
 ]
 NSTATUS = 10
 
@@ -63,6 +65,11 @@ class Timings(ctypes.Structure):
         return dict(h2d_ms=self.h2d_ms, columns_ms=self.columns_ms, pairs_ms=self.pairs_ms,
                     epilogue_ms=self.epilogue_ms, d2h_ms=self.d2h_ms, total_ms=self.total_ms,
                     n_launches=self.n_launches)
+
+
+class EdgeFilter(ctypes.Structure):
+    _fields_ = [("min_abs_cor", ctypes.c_double), ("max_pvalue", ctypes.c_double),
+                ("scale_max", ctypes.c_int32), ("reserved", ctypes.c_int32), ("max_edges", ctypes.c_int64)]
 
 
 class Table(ctypes.Structure):
@@ -151,6 +158,18 @@ def load():
         f = getattr(L, name + "_csc")
         f.argtypes = csc + getattr(L, name).argtypes[4:]
         f.restype = ctypes.c_int
+    L.icikt_all_pairs_edges.argtypes = [_dp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, _dp, ctypes.c_int32,
+                                        ctypes.POINTER(Opts), ctypes.POINTER(EdgeFilter), ctypes.POINTER(vp), _dp,
+                                        ctypes.POINTER(Timings)]
+    L.icikt_all_pairs_edges.restype = ctypes.c_int
+    L.icikt_all_pairs_edges_csc.argtypes = csc + L.icikt_all_pairs_edges.argtypes[4:]
+    L.icikt_all_pairs_edges_csc.restype = ctypes.c_int
+    L.icikt_edges_count.argtypes = [vp]
+    L.icikt_edges_count.restype = ctypes.c_int64
+    L.icikt_edges_copy.argtypes = [vp, _ip, _ip, _dp, _dp, _dp, _dp, _dp]
+    L.icikt_edges_copy.restype = ctypes.c_int
+    L.icikt_edges_free.argtypes = [vp]
+    L.icikt_edges_free.restype = None
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -215,6 +234,13 @@ def is_sparse(x):
 def canonical_csc(x):
     """x as a scipy.sparse CSC matrix or array in canonical format (rows sorted and unique within each
     column).  Duplicate entries are summed, as toarray() does, on a copy: the caller's object stays as it is."""
+    if getattr(x, "format", None) == "csc" and len(x.shape) == 2:
+        # before scipy looks at the arrays: its versions differ in whether, where and with which message they
+        # refuse a column pointer array that disagrees with them
+        nnz = int(x.indptr[-1]) if x.indptr.size else 0
+        if x.indptr.size != x.shape[1] + 1 or x.indices.size < nnz or x.data.size < nnz:
+            raise ValueError(f"malformed CSC matrix: {x.indptr.size} column pointers for {x.shape[1]} columns, "
+                             f"colptr[C] = {nnz}, {x.indices.size} row indices, {x.data.size} values")
     a = x.tocsc()
     if len(a.shape) != 2:
         raise ValueError("data must be a 2-D array (features x samples)")
@@ -305,6 +331,43 @@ def run_pairs(data, global_na=(), pi=None, pj=None, want_counts=False, devices=N
                max_taumax=mx.value, timings=t.as_dict())
     if want_counts:
         out["counts"] = counts
+    return out
+
+
+EDGE_NAMES = ("cor", "raw", "pvalue", "taumax", "completeness")
+
+
+def _bound(v):
+    return float("nan") if v is None else float(v)
+
+
+def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, **opt_kw):
+    """icikt_all_pairs_edges: all pairs, filtered on the device, as a long table of the pairs that pass.
+
+    A pair is kept iff it is not degenerate, abs(cor) >= min_abs_cor and pvalue <= max_pvalue (a bound of None is
+    no condition), with cor = raw / max(taumax over all pairs) if scale_max else raw.  Rows are in the pair order
+    of run_pairs, and every field is bit for bit run_pairs' for that pair.  data may be a scipy.sparse matrix
+    (-> icikt_all_pairs_edges_csc).  max_edges > 0 raises IciktError(ERR_LIMIT) when more pairs pass.
+    Returns a dict of NumPy arrays i, j (int32), cor, raw, pvalue, taumax, completeness, plus max_taumax and
+    timings."""
+    L = load()
+    lead, sfx, n, C, keep_alive = _matrix_args(data)
+    o = make_opts(**opt_kw)
+    f = EdgeFilter(_bound(min_abs_cor), _bound(max_pvalue), int(bool(scale_max)), 0, int(max_edges))
+    h = ctypes.c_void_p()
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(getattr(L, "icikt_all_pairs_edges" + sfx)(*lead, gp, ng, ctypes.byref(o), ctypes.byref(f), ctypes.byref(h),
+                                                    ctypes.byref(mx), ctypes.byref(t)))
+    try:
+        m = int(L.icikt_edges_count(h))
+        out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
+        out.update((k, np.empty(m, dtype=np.float64)) for k in EDGE_NAMES)
+        check(L.icikt_edges_copy(h, _ptr(out["i"]), _ptr(out["j"]), *(_ptr(out[k]) for k in EDGE_NAMES)))
+    finally:
+        L.icikt_edges_free(h)
+    out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 
 

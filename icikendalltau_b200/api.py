@@ -213,6 +213,16 @@ def ici_kt(x, y, perspective="local", alternative="two.sided", continuity=False,
     return res
 
 
+def _edge_mask(cor, pvalue, min_abs_cor, max_pvalue):
+    """rows of a long table that pass the filter of ici_kendalltau (a bound of None is no condition)"""
+    sel = np.ones(len(cor), dtype=bool)
+    if min_abs_cor is not None:
+        sel &= np.abs(cor) >= min_abs_cor
+    if max_pvalue is not None:
+        sel &= pvalue <= max_pvalue
+    return sel
+
+
 def _reshape(names, pi, pj, cols):
     C = len(names)
     out = {}
@@ -226,7 +236,8 @@ def _reshape(names, pi, pj, cols):
 
 def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="global", scale_max=True,
                    diag_good=True, include_only=None, alternative="two.sided", continuity=False,
-                   check_timing=False, return_matrix=True, colnames=None, device=0, n_gpus=1):
+                   check_timing=False, return_matrix=True, colnames=None, device=0, n_gpus=1,
+                   min_abs_cor=None, max_pvalue=None, max_edges=None):
     """All-pairs ICI-Kendall-tau between the columns (samples) of a features x samples matrix.
 
     Returns a dict with `cor`, `raw`, `pvalue`, `taumax`, `completeness` (C x C matrices),
@@ -234,15 +245,30 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     s1, s2, raw, pvalue, taumax, completeness, cor) like the reference's data.frame.
     n_gpus > 1 spreads the pair order over that many GPUs of the box (the role of the reference's
     furrr workers), still in one library call.
+
+    min_abs_cor / max_pvalue (return_matrix=False, one GPU) keep only the rows of the long table with
+    abs(cor) >= min_abs_cor and pvalue <= max_pvalue (a bound of None is no condition; the diagonal rows of
+    diag_good are subject to the same mask).  Over all pairs the selection runs on the device window by window
+    (_lib.run_edges), so neither the result nor the device memory grows with the number of pairs; degenerate
+    pairs never pass and raise no warning there.  max_edges: raise IciktError (ERR_LIMIT) when more computed
+    pairs than that pass.
     """
+    filtered = min_abs_cor is not None or max_pvalue is not None
+    if filtered and return_matrix:
+        raise ValueError("`min_abs_cor` and `max_pvalue` select rows of the long table: pass return_matrix=False")
+    if filtered and n_gpus > 1:
+        raise ValueError("`min_abs_cor` and `max_pvalue` run on one GPU: n_gpus must be 1")
+    if max_edges is not None and not filtered:
+        raise ValueError("`max_edges` limits a filtered table: give `min_abs_cor` or `max_pvalue` too")
     data, names = _colnames_of(data_matrix, colnames, "data_matrix")
     n, C = data.shape
     log.info("Processing missing values ...")
     global_na = [float(v) for v in global_na]
     keep, n_good = _keep_and_n_good(data, global_na)
     log.info("Figuring out comparisons to do ...")
-    if include_only is None and return_matrix and not check_timing:
-        # every pair, in the library's own order, straight into matrices: no pair list on the host
+    if include_only is None and (return_matrix or filtered) and not check_timing:
+        # every pair, in the library's own order, straight into matrices or filtered on the device: no pair
+        # list on the host
         pi = pj = None
         all_pairs = True
         if C < 2 and diag_good:
@@ -284,29 +310,47 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
         out["run_time"] = run_time
         out["names"] = names
         return out
-    if all_pairs and n_gpus > 1:  # one call, the pair order sliced over the GPUs inside the library
-        r = _lib.run_pairs(data, global_na, include_diag=not diag_good, devices=range(n_gpus), **kw)
-    elif all_pairs:
-        r = _lib.run_pairs(data, global_na, include_diag=not diag_good, **kw)
+    if filtered and all_pairs:  # selected on the device, window by window
+        r = _lib.run_edges(data, global_na, min_abs_cor, max_pvalue, scale_max, max_edges or 0,
+                           include_diag=not diag_good, **kw)
+        run_time = time.perf_counter() - t1
+        pi, pj = r["i"], r["j"]
+        raw, pvalue, taumax, completeness, cor = (r[k] for k in ("raw", "pvalue", "taumax", "completeness", "cor"))
     else:
-        r = _lib.run_pairs(data, global_na, pi=pi, pj=pj, **kw)
-    run_time = time.perf_counter() - t1
-    _warn_status(r["status"])
+        if all_pairs and n_gpus > 1:  # one call, the pair order sliced over the GPUs inside the library
+            r = _lib.run_pairs(data, global_na, include_diag=not diag_good, devices=range(n_gpus), **kw)
+        elif all_pairs:
+            r = _lib.run_pairs(data, global_na, include_diag=not diag_good, **kw)
+        else:
+            r = _lib.run_pairs(data, global_na, pi=pi, pj=pj, **kw)
+        run_time = time.perf_counter() - t1
+        _warn_status(r["status"])
 
-    log.info("Recombining results ...")
-    raw, pvalue, taumax, completeness = r["raw"], r["pvalue"], r["taumax"], r["completeness"]
-    if scale_max:  # R/kendalltau.R:368-372: max over the pairs actually computed, na.rm
-        cor = raw / r["max_taumax"]
-    else:
-        cor = raw.copy()
+        log.info("Recombining results ...")
+        raw, pvalue, taumax, completeness = r["raw"], r["pvalue"], r["taumax"], r["completeness"]
+        if scale_max:  # R/kendalltau.R:368-372: max over the pairs actually computed, na.rm
+            cor = raw / r["max_taumax"]
+        else:
+            cor = raw.copy()
+        if filtered:  # include_only: the pair list exists already, the mask runs here
+            sel = _edge_mask(cor, pvalue, min_abs_cor, max_pvalue)
+            if max_edges and int(sel.sum()) > max_edges:
+                raise _lib.IciktError(_lib.ERR_LIMIT, f"more than max_edges = {max_edges} pairs pass the filter "
+                                                      f"({int(sel.sum())})")
+            pi, pj, raw, pvalue, taumax, completeness, cor = (
+                v[sel] for v in (pi, pj, raw, pvalue, taumax, completeness, cor))
     if diag_good:  # R/kendalltau.R:374-386 (appended after scaling, never scaled)
         d = np.arange(C, dtype=np.int32)
         dg = n_good / n_good.max()
+        dp, dt, dc = np.zeros(C), np.ones(C), n_good / n
+        if filtered:
+            sel = _edge_mask(dg, dp, min_abs_cor, max_pvalue)
+            d, dg, dp, dt, dc = d[sel], dg[sel], dp[sel], dt[sel], dc[sel]
         pi, pj = np.concatenate([pi, d]), np.concatenate([pj, d])
         raw, cor = np.concatenate([raw, dg]), np.concatenate([cor, dg])
-        pvalue = np.concatenate([pvalue, np.zeros(C)])
-        taumax = np.concatenate([taumax, np.ones(C)])
-        completeness = np.concatenate([completeness, n_good / n])
+        pvalue = np.concatenate([pvalue, dp])
+        taumax = np.concatenate([taumax, dt])
+        completeness = np.concatenate([completeness, dc])
     if not return_matrix:
         nm = np.asarray(names, dtype=object)
         return dict(cor=dict(s1=nm[pi], s2=nm[pj], raw=raw, pvalue=pvalue, taumax=taumax,

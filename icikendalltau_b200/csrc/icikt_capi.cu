@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "../../include/icikt_b200.h"
+#include "icikt_edges.cuh"
 #include "icikt_internal.h"
 
 using namespace icikt;
@@ -243,6 +244,18 @@ struct icikt_plan {
   std::vector<cudaEvent_t> sync_ev;      // per launch: [2l] its columns have landed, [2l+1] its results are ready
   std::vector<cudaEvent_t> time_ev;      // per launch: K1 start/end, K2 start, K2 end, K3 end
 
+  // Filtered all-pairs call (icikt_all_pairs_edges, see run_edges): the plan's pair buffers hold one window of
+  // the pair order; units, selected rows and the per-window readback are double-buffered.
+  PairUnit* d_wunits[2] = {nullptr, nullptr};
+  PairUnit* h_wunits[2] = {nullptr, nullptr};  // pinned
+  size_t wunit_cap = 0;
+  uint32_t* d_emask = nullptr;
+  uint32_t* d_etile = nullptr;
+  EdgeRow* d_erows[2] = {nullptr, nullptr};
+  unsigned long long* d_etotal = nullptr;  // [2]
+  unsigned long long* h_estat = nullptr;   // pinned [2][2]: rows kept, max taumax bits so far
+  cudaEvent_t eev[2][6]{};                 // per buffer: units up start/end, K2 start, K2 end, K3 end, selection end
+
   cudaEvent_t ev[9]{};
   icikt_timings tm{};
 };
@@ -295,6 +308,17 @@ void free_plan(icikt_plan* p) {
   if (p->h_mat) cudaFreeHost(p->h_mat);
   cudaFree(p->d_hist);
   cudaFree(p->d_ngood);
+  for (int b = 0; b < 2; ++b) {
+    cudaFree(p->d_wunits[b]);
+    if (p->h_wunits[b]) cudaFreeHost(p->h_wunits[b]);
+    cudaFree(p->d_erows[b]);
+    for (auto& e : p->eev[b])
+      if (e) cudaEventDestroy(e);
+  }
+  cudaFree(p->d_emask);
+  cudaFree(p->d_etile);
+  cudaFree(p->d_etotal);
+  if (p->h_estat) cudaFreeHost(p->h_estat);
   for (auto& e : p->ev)
     if (e) cudaEventDestroy(e);
   for (auto& e : p->sync_ev)
@@ -306,6 +330,43 @@ void free_plan(icikt_plan* p) {
   delete p;
 }
 
+// The units of pairs [lo, hi) of the all-pairs order of C columns (combn order, then the diagonal if
+// include_diag), appended to U with slots counted from lo.  `first_row`: a row at or before the row of pair lo
+// (0 always works; the filtered call passes the row of its window).
+void range_units(int64_t C, bool include_diag, int64_t lo, int64_t hi, int64_t slots, std::vector<PairUnit>& U,
+                 int64_t first_row = 0) {
+  const int64_t ptri = tri_pairs(C);
+  int64_t ulen = (hi - lo) / (16 * slots);
+  ulen = std::max<int64_t>(1, std::min<int64_t>(16, ulen));
+  for (int64_t i = first_row; i + 1 < C; ++i) {
+    const int64_t rs = row_start(i, C), re = rs + (C - 1 - i);
+    const int64_t a = std::max(rs, lo), b = std::min(re, hi);
+    for (int64_t s = a; s < b; s += ulen) {
+      PairUnit u;
+      u.slot0 = s - lo;
+      u.col = (int32_t)i;
+      u.j0 = (int32_t)(i + 1 + (s - rs));
+      u.count = (int32_t)std::min<int64_t>(ulen, b - s);
+      u.j_explicit = 0;
+      U.push_back(u);
+    }
+    if (re >= hi) break;
+  }
+  if (include_diag) {
+    for (int64_t i = std::max<int64_t>(0, lo - ptri); i < C; ++i) {
+      const int64_t s = ptri + i;
+      if (s < lo || s >= hi) continue;
+      PairUnit u;
+      u.slot0 = s - lo;
+      u.col = (int32_t)i;
+      u.j0 = (int32_t)i;
+      u.count = 1;
+      u.j_explicit = 0;
+      U.push_back(u);
+    }
+  }
+}
+
 // Split the pair order into units: consecutive pairs that share their first column.
 int build_units(icikt_plan* p, const int32_t* pi, const int32_t* pj, int64_t P_list) {
   const int64_t C = p->C;
@@ -313,41 +374,12 @@ int build_units(icikt_plan* p, const int32_t* pi, const int32_t* pj, int64_t P_l
   U.clear();
   const int64_t slots = (int64_t)p->n_sm * 2;
   if (!pi) {
-    const int64_t ptri = tri_pairs(C);
-    const int64_t ptot = ptri + (p->opts.include_diag ? C : 0);
+    const int64_t ptot = tri_pairs(C) + (p->opts.include_diag ? C : 0);
     int64_t lo = p->opts.pair_lo, hi = p->opts.pair_hi;
     if (lo == 0 && hi == 0) hi = ptot;
     if (lo < 0 || hi > ptot || lo > hi) return fail(ICIKT_ERR_BAD_ARG, "pair_lo/pair_hi out of range");
     p->P = hi - lo;
-    int64_t ulen = p->P / (16 * slots);
-    ulen = std::max<int64_t>(1, std::min<int64_t>(16, ulen));
-    for (int64_t i = 0; i + 1 < C; ++i) {
-      const int64_t rs = row_start(i, C), re = rs + (C - 1 - i);
-      const int64_t a = std::max(rs, lo), b = std::min(re, hi);
-      for (int64_t s = a; s < b; s += ulen) {
-        PairUnit u;
-        u.slot0 = s - lo;
-        u.col = (int32_t)i;
-        u.j0 = (int32_t)(i + 1 + (s - rs));
-        u.count = (int32_t)std::min<int64_t>(ulen, b - s);
-        u.j_explicit = 0;
-        U.push_back(u);
-      }
-      if (re >= hi) break;
-    }
-    if (p->opts.include_diag) {
-      for (int64_t i = 0; i < C; ++i) {
-        const int64_t s = ptri + i;
-        if (s < lo || s >= hi) continue;
-        PairUnit u;
-        u.slot0 = s - lo;
-        u.col = (int32_t)i;
-        u.j0 = (int32_t)i;
-        u.count = 1;
-        u.j_explicit = 0;
-        U.push_back(u);
-      }
-    }
+    range_units(C, p->opts.include_diag != 0, lo, hi, slots, U);
   } else {
     p->P = P_list;
     for (int64_t k = 0; k < P_list; ++k)
@@ -992,15 +1024,16 @@ int icikt_plan_tables(icikt_plan* p, icikt_table* out, int32_t cap) {
   return n_out;
 }
 
-// K2 (every tier's shape; the device-side maxima pick the one that runs) + K3 over units [unit_lo, unit_hi);
-// e_start / e_mid / e_end bracket K2 and K3 on the plan's stream
-static int launch_pair_group(icikt_plan* p, int64_t unit_lo, int64_t unit_hi, int max_unit_pairs, cudaEvent_t e_start,
+// K2 (every tier's shape; the device-side maxima pick the one that runs) + K3 over units [unit_lo, unit_hi) of
+// `units` (device; the plan's own table unless the filtered call passes a window's); e_start / e_mid / e_end
+// bracket K2 and K3 on the plan's stream
+static int launch_pair_group(icikt_plan* p, const PairUnit* units, int64_t unit_lo, int64_t unit_hi, int max_unit_pairs, cudaEvent_t e_start,
                              cudaEvent_t e_mid, cudaEvent_t e_end, int* launches_out) {
   CK(cudaMemsetAsync(p->d_scalars, 0, 2 * sizeof(unsigned long long), p->stream));
   CK(cudaEventRecord(e_start, p->stream));
   PairLaunch pl;
   pl.tab = &p->tab;
-  pl.units = p->d_units + unit_lo;
+  pl.units = units + unit_lo;
   pl.n_units = unit_hi - unit_lo;
   pl.pj_list = p->d_pj;
   pl.raw = p->d_raw;
@@ -1065,7 +1098,7 @@ int icikt_plan_pairs(icikt_plan* p) {
   CK(cudaSetDevice(p->device));
   CK(cudaMemsetAsync(p->d_maxbits, 0, sizeof(unsigned long long), p->stream));
   int launches = 0;
-  const int rc = launch_pair_group(p, 0, (int64_t)p->units.size(), p->max_unit_pairs, p->ev[4], p->ev[8], p->ev[5], &launches);
+  const int rc = launch_pair_group(p, p->d_units, 0, (int64_t)p->units.size(), p->max_unit_pairs, p->ev[4], p->ev[8], p->ev[5], &launches);
   if (rc != ICIKT_OK) return rc;
   p->tm.n_launches = (p->tm.n_launches & 0xffff) | (launches << 16);
   p->pairs_done = true;
@@ -1296,7 +1329,7 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
       rc = plan_columns_impl(p, global_na, n_global_na, st.col_lo, st.col_hi, st.col_hi == p->C, st.col_lo == 0, te[0], te[1]);
       if (rc != ICIKT_OK) return rc;
     }
-    const int rc = launch_pair_group(p, st.unit_lo, st.unit_hi, st.max_unit_pairs, te[2], te[3], te[4], &pair_launches);
+    const int rc = launch_pair_group(p, p->d_units, st.unit_lo, st.unit_hi, st.max_unit_pairs, te[2], te[3], te[4], &pair_launches);
     if (rc != ICIKT_OK) return rc;
     CK(cudaEventRecord(p->sync_ev[2 * l + 1], p->stream));
   }
@@ -1386,6 +1419,7 @@ static bool want_staged(int64_t n, int64_t C, const icikt_opts& o, bool all_pair
 // One cached plan for the one-shot entry points (all-pairs shape only).
 static icikt_plan* g_cached = nullptr;
 static icikt_plan* g_cached_multi[64] = {};  // one slot per worker of icikt_all_pairs_multi
+static icikt_plan* g_cached_edges = nullptr;    // the filtered call's (its pair buffers hold one window)
 static std::mutex g_cache_mu;
 
 static bool cache_matches(const icikt_plan* p, int64_t n, int64_t C, const icikt_opts& o, bool staged) {
@@ -1476,6 +1510,7 @@ int icikt_pair_from_index(int64_t C, int32_t include_diag, int64_t index, int32_
 void icikt_release_workspace(void) {
   std::lock_guard<std::mutex> lock(g_cache_mu);
   if (g_cached) { icikt_plan_destroy(g_cached); g_cached = nullptr; }
+  if (g_cached_edges) { icikt_plan_destroy(g_cached_edges); g_cached_edges = nullptr; }
   for (icikt_plan*& s : g_cached_multi)
     if (s) { icikt_plan_destroy(s); s = nullptr; }
 }
@@ -1594,6 +1629,322 @@ int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const doubl
   return matrices_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max,
                        diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
 }
+
+}  // extern "C"
+
+// ---- all pairs, filtered on the device (icikt_all_pairs_edges) ------------------------------------------------
+
+struct icikt_edges {
+  std::vector<EdgeRow> rows;
+  std::vector<double> cor;
+};
+
+// Pairs per window of the filtered call (ICIKT_EDGE_WINDOW, at most 2^30).  The default 2^26 keeps the window's
+// buffers near 10 GB: the plan's pair buffers (68 B per pair) and the two selected-row buffers (40 B each).
+static int64_t edge_window() {
+  const char* e = std::getenv("ICIKT_EDGE_WINDOW");
+  const long long v = e ? std::atoll(e) : 0;
+  return v > 0 ? std::min<long long>(v, 1LL << 30) : (1LL << 26);
+}
+
+static double max_of_bits(unsigned long long bits) {
+  double v;
+  std::memcpy(&v, &bits, sizeof(v));
+  return bits ? v : std::nan("");
+}
+
+// The argument checks of the filtered call, on the host before any device is touched.
+static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                           const icikt_opts& o, const icikt_edge_filter* f, icikt_edges** out) {
+  if (!out) return fail(ICIKT_ERR_BAD_ARG, "out is NULL");
+  *out = nullptr;
+  if (!f) return fail(ICIKT_ERR_BAD_ARG, "filter is NULL");
+  if (f->max_edges < 0) return fail(ICIKT_ERR_BAD_ARG, "max_edges must be >= 0 (0: no limit)");
+  if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
+  if (!s.csc() && (!s.data || s.ld < n)) return fail(ICIKT_ERR_BAD_ARG, "data must not be NULL and ld >= n");
+  if (n > tiled_max_n()) return fail(ICIKT_ERR_TOO_LONG, "n exceeds icikt_max_n()");
+  if (C > 2147483647LL) return fail(ICIKT_ERR_BAD_ARG, "too many columns");
+  if (n_global_na < 0 || (n_global_na > 0 && !global_na)) return fail(ICIKT_ERR_BAD_ARG, "bad global_na");
+  if (o.pair_lo != 0 || o.pair_hi != 0)
+    return fail(ICIKT_ERR_BAD_ARG, "the filtered call covers all pairs: pair_lo and pair_hi must be 0");
+  if (o.perspective != ICIKT_PERSPECTIVE_GLOBAL && o.perspective != ICIKT_PERSPECTIVE_LOCAL)
+    return fail(ICIKT_ERR_BAD_ARG, "the filtered call takes the global or the local perspective");
+  if (o.kernel != ICIKT_KERNEL_TILED) return fail(ICIKT_ERR_BAD_ARG, "the filtered call needs the tiled kernel");
+  if (o.want_counts) return fail(ICIKT_ERR_BAD_ARG, "the filtered call returns no counts (want_counts)");
+  return ICIKT_OK;
+}
+
+#define ECK(call)                                                                                              \
+  do {                                                                                                         \
+    cudaError_t e_ = (call);                                                                                   \
+    if (e_ != cudaSuccess)                                                                                     \
+      return e_ == cudaErrorMemoryAllocation ? (cudaGetLastError(), fail(ICIKT_ERR_ALLOC, "allocation failed: " #call)) \
+                                             : cuda_fail(e_, #call);                                           \
+  } while (0)
+
+// the selection's buffers for windows of W pairs (kept with the plan)
+static int ensure_edge_buffers(icikt_plan* p, int64_t W) {
+  if (p->d_etotal) return ICIKT_OK;
+  const int64_t tiles = (W + kEdgeTile - 1) / kEdgeTile;
+  if (!p->copy_stream) ECK(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
+  ECK(dmalloc(&p->d_emask, (size_t)tiles * (kEdgeTile / 32)));
+  ECK(dmalloc(&p->d_etile, (size_t)tiles));
+  for (int b = 0; b < 2; ++b) {
+    ECK(dmalloc(&p->d_erows[b], (size_t)W));
+    for (auto& e : p->eev[b]) ECK(cudaEventCreate(&e));
+  }
+  ECK(cudaMallocHost(reinterpret_cast<void**>(&p->h_estat), 4 * sizeof(unsigned long long)));
+  ECK(dmalloc(&p->d_etotal, 2));
+  return ensure_stage(p);
+}
+
+// room for `need` units in both window unit buffers (device and pinned host)
+static int ensure_window_units(icikt_plan* p, size_t need) {
+  if (need <= p->wunit_cap) return ICIKT_OK;
+  CK(cudaStreamSynchronize(p->stream));  // the other buffer may still be read by the previous window
+  const size_t cap = std::max(need + need / 4, 2 * p->wunit_cap);
+  for (int b = 0; b < 2; ++b) {
+    cudaFree(p->d_wunits[b]);
+    if (p->h_wunits[b]) cudaFreeHost(p->h_wunits[b]);
+    p->d_wunits[b] = nullptr;
+    p->h_wunits[b] = nullptr;
+  }
+  p->wunit_cap = 0;
+  for (int b = 0; b < 2; ++b) {
+    ECK(dmalloc(&p->d_wunits[b], cap));
+    ECK(cudaMallocHost(reinterpret_cast<void**>(&p->h_wunits[b]), sizeof(PairUnit) * cap));
+  }
+  p->wunit_cap = cap;
+  return ICIKT_OK;
+}
+
+// The filtered call on a plan whose pair buffers hold W pairs: upload and K1 once, then the pair order in windows
+// of W.  Window w is enqueued (units, K2, K3, selection, the readback of its row count and of the maximum so far)
+// before the host waits for window w - 1, copies its rows out on the copy stream and re-trims the rows it holds
+// against the new maximum; d_maxbits is not reset between windows, so K3's atomicMax leaves that maximum.
+static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
+                        const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
+                        icikt_timings* timings) {
+  int rc = ensure_edge_buffers(p, W);
+  if (rc == ICIKT_OK) rc = upload_columns(p, s, 0, p->C);
+  if (rc == ICIKT_OK) rc = plan_columns_impl(p, global_na, n_global_na, 0, p->C, true);
+  if (rc != ICIKT_OK) return rc;
+  int launches = p->tm.n_launches;
+  CK(cudaMemsetAsync(p->d_maxbits, 0, sizeof(unsigned long long), p->stream));
+  const double t = f.min_abs_cor;
+  const bool scale = f.scale_max != 0;
+  const bool retrim = scale && t == t;
+  const int64_t nwin = (ptot + W - 1) / W, ptri = tri_pairs(p->C), slots = (int64_t)p->n_sm * 2;
+  std::vector<PairUnit> U;
+  std::vector<EdgeRow>& rows = res->rows;
+  float up_ms = 0.f, pairs_ms = 0.f, epi_ms = 0.f, d2h_ms = 0.f;
+  unsigned long long bits = 0, trimmed_bits = 0;
+
+  auto enqueue = [&](int64_t w) -> int {
+    const int b = (int)(w & 1);
+    const int64_t lo = w * W, hi = std::min(ptot, lo + W);
+    int32_t row = 0, col = 0;
+    if (lo < ptri) icikt_pair_from_index(p->C, 0, lo, &row, &col);
+    U.clear();
+    range_units(p->C, p->opts.include_diag != 0, lo, hi, slots, U, row);
+    int r = ensure_window_units(p, U.size());
+    if (r != ICIKT_OK) return r;
+    // the buffer was last read by window w - 2, whose selection the host has waited for
+    std::memcpy(p->h_wunits[b], U.data(), sizeof(PairUnit) * U.size());
+    int max_unit = 1;
+    for (const PairUnit& u : U) max_unit = std::max(max_unit, (int)u.count);
+    cudaEvent_t* e = p->eev[b];
+    CK(cudaEventRecord(e[0], p->stream));
+    CK(cudaMemcpyAsync(p->d_wunits[b], p->h_wunits[b], sizeof(PairUnit) * U.size(), cudaMemcpyHostToDevice, p->stream));
+    CK(cudaEventRecord(e[1], p->stream));
+    r = launch_pair_group(p, p->d_wunits[b], 0, (int64_t)U.size(), max_unit, e[2], e[3], e[4], &launches);
+    if (r != ICIKT_OK) return r;
+    EdgeSelect es;
+    es.units = p->d_wunits[b];
+    es.n_units = (int64_t)U.size();
+    es.n_slots = hi - lo;
+    es.tau = p->d_tau;
+    es.pvalue = p->d_p;
+    es.taumax = p->d_tm;
+    es.completeness = p->d_comp;
+    es.status = p->d_status;
+    es.max_taumax_bits = p->d_maxbits;
+    es.min_abs_cor = f.min_abs_cor;
+    es.max_pvalue = f.max_pvalue;
+    es.scale_max = scale ? 1 : 0;
+    es.mask = p->d_emask;
+    es.tile_offset = p->d_etile;
+    es.total = p->d_etotal + b;
+    es.rows = p->d_erows[b];
+    const int l = launch_edge_select(es, p->stream);
+    if (l < 0) return launch_fail("edge selection kernels");
+    launches += l;
+    CK(cudaMemcpyAsync(p->h_estat + 2 * b, p->d_etotal + b, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaMemcpyAsync(p->h_estat + 2 * b + 1, p->d_maxbits, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaEventRecord(e[5], p->stream));
+    return ICIKT_OK;
+  };
+
+  auto collect = [&](int64_t w) -> int {
+    const int b = (int)(w & 1);
+    cudaEvent_t* e = p->eev[b];
+    CK(cudaEventSynchronize(e[5]));
+    const unsigned long long cnt = p->h_estat[2 * b];
+    bits = p->h_estat[2 * b + 1];
+    up_ms += ev_ms(e[0], e[1]);
+    pairs_ms += ev_ms(e[2], e[3]);
+    epi_ms += ev_ms(e[3], e[5]);
+    if (cnt) {
+      const size_t old = rows.size();
+      try {
+        rows.resize(old + (size_t)cnt);
+      } catch (const std::bad_alloc&) {
+        return fail(ICIKT_ERR_ALLOC, "out of host memory for the selected rows");
+      }
+      CK(cudaEventRecord(p->ev[6], p->copy_stream));
+      const int r = staged_copy_out(p, rows.data() + old, p->d_erows[b], sizeof(EdgeRow) * (size_t)cnt, p->copy_stream);
+      if (r != ICIKT_OK) return r;
+      CK(cudaEventRecord(p->ev[7], p->copy_stream));
+      CK(cudaEventSynchronize(p->ev[7]));
+      d2h_ms += ev_ms(p->ev[6], p->ev[7]);
+    }
+    if (retrim && bits != trimmed_bits) {  // the maximum grew: rows held from earlier windows may no longer pass
+      const double m = max_of_bits(bits);
+      rows.erase(std::remove_if(rows.begin(), rows.end(), [&](const EdgeRow& r) { return !edge_prefilter(r.raw, t, m); }),
+                 rows.end());
+      trimmed_bits = bits;
+    }
+    if (f.max_edges > 0 && (int64_t)rows.size() > f.max_edges)
+      return fail(ICIKT_ERR_LIMIT, "more than max_edges = " + std::to_string(f.max_edges) + " pairs pass the filter (" +
+                                       std::to_string(rows.size()) + " held after " + std::to_string(w + 1) + " of " +
+                                       std::to_string(nwin) + " windows)");
+    return ICIKT_OK;
+  };
+
+  for (int64_t w = 0; w <= nwin; ++w) {
+    if (w < nwin && (rc = enqueue(w)) != ICIKT_OK) return rc;
+    if (w > 0 && (rc = collect(w - 1)) != ICIKT_OK) return rc;
+  }
+  // the exact predicate with the final maximum
+  const double M = max_of_bits(bits);
+  if (scale && t == t)
+    rows.erase(std::remove_if(rows.begin(), rows.end(), [&](const EdgeRow& r) { return !edge_keep_final(r.raw, t, true, M); }),
+               rows.end());
+  if (f.max_edges > 0 && (int64_t)rows.size() > f.max_edges)
+    return fail(ICIKT_ERR_LIMIT, "more than max_edges = " + std::to_string(f.max_edges) + " pairs pass the filter (" +
+                                     std::to_string(rows.size()) + ")");
+  res->cor.resize(rows.size());
+  for (size_t k = 0; k < rows.size(); ++k) res->cor[k] = scale ? rows[k].raw / M : rows[k].raw;
+  CK(cudaEventRecord(p->ev[4], p->copy_stream));
+  CK(cudaStreamWaitEvent(p->stream, p->ev[4], 0));
+  CK(cudaEventRecord(p->ev[5], p->stream));
+  CK(cudaEventSynchronize(p->ev[5]));
+  if (max_taumax) *max_taumax = M;
+  if (timings) {
+    std::memset(timings, 0, sizeof(*timings));
+    timings->h2d_ms = ev_ms(p->ev[0], p->ev[1]) + up_ms;
+    timings->columns_ms = ev_ms(p->ev[2], p->ev[3]);
+    timings->pairs_ms = pairs_ms;
+    timings->epilogue_ms = epi_ms;
+    timings->d2h_ms = d2h_ms;
+    timings->total_ms = ev_ms(p->ev[0], p->ev[5]);
+    timings->n_launches = launches;
+    cudaGetLastError();
+  }
+  return ICIKT_OK;
+}
+#undef ECK
+
+static int all_pairs_edges(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                           const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
+                           double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  int rc = check_edge_args(s, n, C, global_na, n_global_na, o, filter, out);
+  if (rc != ICIKT_OK) return rc;
+  rc = select_device(o.device);
+  if (rc != ICIKT_OK) return rc;
+  icikt_edges* res = new (std::nothrow) icikt_edges();
+  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
+  const int64_t ptot = tri_pairs(C) + (o.include_diag ? C : 0);
+  if (ptot == 0) {  // one column, no diagonal: nothing to compute
+    if (max_taumax) *max_taumax = std::nan("");
+    if (timings) std::memset(timings, 0, sizeof(*timings));
+    *out = res;
+    return ICIKT_OK;
+  }
+  const int64_t W = std::min(edge_window(), ptot);
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  icikt_plan* p = g_cached_edges;
+  if (p && p->n == n && p->C == C && p->P == W && p->opts.device == o.device && p->opts.include_diag == o.include_diag) {
+    p->opts.perspective = o.perspective;
+    p->opts.alternative = o.alternative;
+    p->opts.continuity = o.continuity;
+    p->opts.na_inf = o.na_inf;
+  } else {
+    if (p) icikt_plan_destroy(p);
+    g_cached_edges = nullptr;
+    icikt_opts po = o;
+    po.pair_hi = W;  // the plan's pair buffers: one window
+    rc = plan_create_impl(&p, n, C, nullptr, nullptr, 0, &po, false);
+    if (rc != ICIKT_OK) {
+      delete res;
+      return rc;
+    }
+    g_cached_edges = p;
+  }
+  rc = edge_windows(p, s, global_na, n_global_na, *filter, ptot, W, res, max_taumax, timings);
+  if (rc != ICIKT_OK) {
+    const std::string keep = g_err;
+    icikt_plan_destroy(g_cached_edges);  // waits for whatever the failed call left in flight
+    g_cached_edges = nullptr;
+    delete res;
+    g_err = keep;
+    return rc;
+  }
+  *out = res;
+  return ICIKT_OK;
+}
+
+extern "C" {
+
+int icikt_all_pairs_edges(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                          int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
+                          icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  return all_pairs_edges(dense_source(data, ld), n, C, global_na, n_global_na, opts, filter, out, max_taumax, timings);
+}
+
+int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                              int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                              const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                              icikt_timings* timings) {
+  if (out) *out = nullptr;
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return all_pairs_edges(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, filter, out,
+                         max_taumax, timings);
+}
+
+int64_t icikt_edges_count(const icikt_edges* e) { return e ? (int64_t)e->rows.size() : 0; }
+
+int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, double* raw, double* pvalue,
+                     double* taumax, double* completeness) {
+  if (!e) return fail(ICIKT_ERR_BAD_ARG, "edges is NULL");
+  const size_t m = e->rows.size();
+  for (size_t k = 0; k < m; ++k) {
+    const EdgeRow& r = e->rows[k];
+    if (i) i[k] = r.i;
+    if (j) j[k] = r.j;
+    if (raw) raw[k] = r.raw;
+    if (pvalue) pvalue[k] = r.pvalue;
+    if (taumax) taumax[k] = r.taumax;
+    if (completeness) completeness[k] = r.completeness;
+  }
+  if (cor && m) std::memcpy(cor, e->cor.data(), sizeof(double) * m);
+  return ICIKT_OK;
+}
+
+void icikt_edges_free(icikt_edges* e) { delete e; }
 
 }  // extern "C"
 

@@ -201,6 +201,29 @@ int launch_missing_matrix(const uint32_t* bits, int64_t words, int64_t n, int64_
 int launch_csc_expand(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t c_lo,
                       int64_t c_hi, double* out, cudaStream_t stream);
 
+// The selection of the filtered all-pairs call (icikt_select.cu): an order-preserving compaction of one window
+// of the pair order.  Tiles of kEdgeTile slots: a count pass writes one ballot word per 32 slots and the kept
+// rows per tile, one CTA turns the tile counts into exclusive offsets (and `total`), and a scatter pass writes
+// the kept slots as EdgeRow (icikt_edges.cuh) in pair order, (i, j) taken from the window's units.
+struct EdgeRow;
+constexpr int kEdgeTile = 1024;
+struct EdgeSelect {
+  const PairUnit* units;  // device, the window's units (slots relative to the window)
+  int64_t n_units;
+  int64_t n_slots;        // pairs in the window
+  const double *tau, *pvalue;
+  const double *taumax, *completeness;
+  const int32_t* status;
+  const unsigned long long* max_taumax_bits;  // the maximum so far (K3 of this window has run)
+  double min_abs_cor, max_pvalue;             // NaN: no condition
+  int scale_max;
+  uint32_t* mask;         // device [n_tiles * kEdgeTile / 32]
+  uint32_t* tile_offset;  // device [n_tiles]
+  unsigned long long* total;  // device, rows kept
+  EdgeRow* rows;          // device [n_slots]
+};
+int launch_edge_select(const EdgeSelect& s, cudaStream_t stream);
+
 int launch_pnorm(const double* d_z, int64_t n, int lower, double* d_out, cudaStream_t stream);
 
 int64_t tiled_max_n();

@@ -1,0 +1,171 @@
+// icikt_select.cu -- the selection of the filtered all-pairs call (icikt_all_pairs_edges): an order-preserving
+// compaction of one window of the pair order, deterministic, in three kernels:
+//   * edge_count_kernel: one CTA per tile of kEdgeTile slots; a warp ballot of the predicate is one mask word
+//     per 32 slots, the popcounts summed over the CTA are the tile's count;
+//   * edge_scan_kernel: one CTA, the tile counts -> exclusive offsets in place, and the total;
+//   * edge_scatter_kernel: one CTA per tile; a tile's 32 mask words are its slots in pair order, so one warp scan
+//     over their popcounts gives every word's offset and a kept slot's rank within its word is a popc of the
+//     bits below it.  Tiles without a kept slot stop after reading their 32 words.
+// HBM-bound: the count pass reads the status and, only for a bound that is given, raw (8 B) and the p-value
+// (8 B); the scatter pass reads 1/8 B of mask per slot and the fields of the kept slots.
+#include "icikt_edges.cuh"
+#include "icikt_internal.h"
+
+namespace icikt {
+
+namespace {
+
+constexpr unsigned FULL = 0xffffffffu;
+constexpr int kSelThreads = 256;
+constexpr int kSelRounds = kEdgeTile / kSelThreads;  // slots per thread
+static_assert(kEdgeTile / 32 == 32, "a tile's mask words are scanned by one warp");
+
+__device__ __forceinline__ double max_so_far(const unsigned long long* bits) {
+  const unsigned long long b = *bits;
+  return b ? __longlong_as_double((long long)b) : __longlong_as_double(0x7ff8000000000000LL);
+}
+
+__global__ void __launch_bounds__(kSelThreads) edge_count_kernel(const EdgeSelect s) {
+  __shared__ unsigned warp_sum[kSelThreads / 32];
+  const long long tile = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const double m = s.scale_max ? max_so_far(s.max_taumax_bits) : 1.0;
+  const bool use_t = s.min_abs_cor == s.min_abs_cor, use_a = s.max_pvalue == s.max_pvalue;
+  unsigned cnt = 0;
+#pragma unroll
+  for (int k = 0; k < kSelRounds; ++k) {
+    const long long slot = tile * kEdgeTile + k * kSelThreads + threadIdx.x;
+    bool keep = false;
+    if (slot < s.n_slots) {
+      const int32_t st = s.status[slot];
+      if (st == 0) {
+        const double raw = use_t ? s.tau[slot] : 0.0;
+        const double pv = use_a ? s.pvalue[slot] : 0.0;
+        keep = edge_keep_window(st, raw, pv, s.min_abs_cor, s.max_pvalue, s.scale_max != 0, m);
+      }
+    }
+    const unsigned word = __ballot_sync(FULL, keep);
+    if (lane == 0) s.mask[(tile * kEdgeTile + k * kSelThreads) / 32 + warp] = word;
+    cnt += __popc(word);
+  }
+  if (lane == 0) warp_sum[warp] = cnt;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned t = 0;
+#pragma unroll
+    for (int w = 0; w < kSelThreads / 32; ++w) t += warp_sum[w];
+    s.tile_offset[tile] = t;
+  }
+}
+
+// exclusive scan of n tile counts in place; one CTA of 1024 threads, each owns a contiguous run of tiles
+__global__ void __launch_bounds__(1024) edge_scan_kernel(uint32_t* __restrict__ v, long long n,
+                                                         unsigned long long* __restrict__ total) {
+  __shared__ unsigned long long warp_tot[32];
+  const long long per = (n + 1023) / 1024;
+  const long long lo = min(n, per * threadIdx.x), hi = min(n, lo + per);
+  unsigned long long sum = 0;
+  for (long long k = lo; k < hi; ++k) sum += v[k];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned long long incl = sum;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const unsigned long long o = __shfl_up_sync(FULL, incl, d);
+    if (lane >= d) incl += o;
+  }
+  if (lane == 31) warp_tot[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    unsigned long long w = warp_tot[lane], wi = w;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const unsigned long long o = __shfl_up_sync(FULL, wi, d);
+      if (lane >= d) wi += o;
+    }
+    warp_tot[lane] = wi - w;  // exclusive over the warps
+    if (lane == 31) *total = wi;
+  }
+  __syncthreads();
+  unsigned long long run = warp_tot[warp] + incl - sum;
+  for (long long k = lo; k < hi; ++k) {
+    const unsigned c = v[k];
+    v[k] = (uint32_t)run;
+    run += c;
+  }
+}
+
+// last unit of [a, b) whose first slot is <= slot (units are in slot order and the first one starts at or
+// before it)
+__device__ __forceinline__ long long unit_of(const PairUnit* __restrict__ units, long long a, long long b,
+                                             long long slot) {
+  while (b - a > 1) {
+    const long long mid = (a + b) >> 1;
+    if (units[mid].slot0 <= slot) a = mid; else b = mid;
+  }
+  return a;
+}
+
+__global__ void __launch_bounds__(kSelThreads) edge_scatter_kernel(const EdgeSelect s) {
+  __shared__ uint32_t words[32];
+  __shared__ uint32_t word_off[32];
+  __shared__ long long unit_range[2];
+  const long long tile = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (warp == 0) {
+    const uint32_t w = s.mask[tile * 32 + lane];
+    const unsigned c = __popc(w);
+    unsigned incl = c;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const unsigned o = __shfl_up_sync(FULL, incl, d);
+      if (lane >= d) incl += o;
+    }
+    words[lane] = w;
+    word_off[lane] = incl - c;
+    if (lane == 31) unit_range[0] = incl;  // the tile's count, for the early exit
+  }
+  __syncthreads();
+  if (unit_range[0] == 0) return;
+  __syncthreads();
+  if (threadIdx.x < 2) {  // the units that cover the tile: [first, last]
+    const long long first_slot = tile * kEdgeTile;
+    const long long last_slot = min((long long)s.n_slots, first_slot + kEdgeTile) - 1;
+    unit_range[threadIdx.x] = unit_of(s.units, 0, s.n_units, threadIdx.x ? last_slot : first_slot);
+  }
+  __syncthreads();
+  const long long ua = unit_range[0], ub = unit_range[1] + 1;
+  const unsigned base = s.tile_offset[tile];
+#pragma unroll
+  for (int k = 0; k < kSelRounds; ++k) {
+    const int m = k * (kSelThreads / 32) + warp;
+    const uint32_t w = words[m];
+    if (!((w >> lane) & 1u)) continue;
+    const long long slot = tile * kEdgeTile + m * 32 + lane;
+    const PairUnit u = s.units[unit_of(s.units, ua, ub, slot)];
+    EdgeRow r;
+    r.i = u.col;
+    r.j = u.j0 + (int32_t)(slot - u.slot0);
+    r.raw = s.tau[slot];
+    r.pvalue = s.pvalue[slot];
+    r.taumax = s.taumax[slot];
+    r.completeness = s.completeness[slot];
+    s.rows[base + word_off[m] + __popc(w & ((1u << lane) - 1u))] = r;
+  }
+}
+
+}  // namespace
+
+int launch_edge_select(const EdgeSelect& s, cudaStream_t stream) {
+  if (s.n_slots <= 0) {
+    cudaMemsetAsync(s.total, 0, sizeof(unsigned long long), stream);
+    return launch_status(0);
+  }
+  const long long tiles = (s.n_slots + kEdgeTile - 1) / kEdgeTile;
+  if (tiles > 0x7fffffffLL) return launch_refused("edge selection: window too large");
+  edge_count_kernel<<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  edge_scan_kernel<<<1, 1024, 0, stream>>>(s.tile_offset, tiles, s.total);
+  edge_scatter_kernel<<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  return launch_status(3);
+}
+
+}  // namespace icikt

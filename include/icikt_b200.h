@@ -49,6 +49,7 @@ extern "C" {
 #define ICIKT_ERR_TOO_LONG (-3)   /* n > icikt_max_n()                                     */
 #define ICIKT_ERR_CUDA (-4)       /* CUDA runtime failure, see icikt_last_error()          */
 #define ICIKT_ERR_ALLOC (-5)      /* host or device allocation failed                      */
+#define ICIKT_ERR_LIMIT (-6)      /* more pairs pass an edge filter than its max_edges     */
 
 /* per-pair status (src/kendallc.cpp line of the matching early return) */
 #define ICIKT_STATUS_OK 0
@@ -228,6 +229,51 @@ int icikt_pairwise_completeness_csc(const int64_t* colptr, const int32_t* rowidx
                                     int32_t n_global_na, int32_t device, const int32_t* pi,
                                     const int32_t* pj, int64_t P, int32_t* missing,
                                     double* completeness, double* matrix);
+
+/* ---- all pairs, filtered on the device: only the pairs that pass a correlation or p-value threshold (the
+ * network of a wide matrix) come back, as a long table in host memory owned by the library.  Device memory
+ * does not depend on the number of pairs P: it is the per-column tables plus one window of W pairs of the
+ * pair order (ICIKT_EDGE_WINDOW, default 2^26), which is computed, filtered and copied out while the next
+ * window runs.  A pair is an edge iff
+ *
+ *   status == 0  &&  (isnan(min_abs_cor) || fabs(cor) >= min_abs_cor)  &&  (isnan(max_pvalue) || pvalue <= max_pvalue)
+ *
+ * with cor = scale_max ? raw / M : raw, M = max(taumax) over ALL computed pairs (the IEEE division of
+ * icikt_plan_download_matrices).  A NaN bound is no condition.  Edges are in the pair order of icikt_all_pairs
+ * (combn order, then the diagonal if include_diag), and every field is bit for bit what icikt_all_pairs
+ * returns for that pair: the result is the full per-pair result, masked.
+ * Options: perspective global or local, alternative, continuity, na_inf, device, include_diag.  Refused with
+ * ICIKT_ERR_BAD_ARG before any device is touched: pair_lo / pair_hi != 0, ICIKT_PERSPECTIVE_COMPLETE,
+ * ICIKT_KERNEL_NAIVE, want_counts, max_edges < 0, a NULL filter or out.  max_edges > 0 fails the call with
+ * ICIKT_ERR_LIMIT once more rows than that are held; with scale_max that count is taken after each window
+ * against the maximum so far, so it may include rows the final maximum removes.  On success *out receives
+ * the rows (free with icikt_edges_free), max_taumax (may be NULL) M or NaN.  timings (may be NULL): pairs_ms
+ * is the sum of K2 over the windows, epilogue_ms of K3 and the selection, h2d_ms / d2h_ms cover their copies. */
+typedef struct icikt_edge_filter {
+  double min_abs_cor; /* NaN: no condition on cor                                     */
+  double max_pvalue;  /* NaN: no condition on the p-value                             */
+  int32_t scale_max;  /* cor = raw / max(taumax) over all pairs, or raw               */
+  int32_t reserved;   /* 0                                                            */
+  int64_t max_edges;  /* 0: no limit; otherwise fail with ICIKT_ERR_LIMIT             */
+} icikt_edge_filter;
+
+typedef struct icikt_edges icikt_edges; /* result rows in host memory owned by the library */
+
+int icikt_all_pairs_edges(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                          int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
+                          icikt_edges** out, double* max_taumax, icikt_timings* timings);
+/* the same for a CSC matrix (see the sparse calls above) */
+int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                              int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                              const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                              icikt_timings* timings);
+/* number of rows (0 for NULL) */
+int64_t icikt_edges_count(const icikt_edges* e);
+/* the rows into caller arrays of icikt_edges_count(e) entries; any pointer may be NULL.  i < j, or i == j for
+ * the diagonal pairs; cor as defined above */
+int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, double* raw, double* pvalue,
+                     double* taumax, double* completeness);
+void icikt_edges_free(icikt_edges* e);
 
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
