@@ -17,6 +17,8 @@ LIB_PATH = os.environ.get("ICIKT_LIB_PATH") or os.path.join(_HERE, "libicikt_b20
 OK = 0
 ERR_NO_DEVICE, ERR_BAD_ARG, ERR_TOO_LONG, ERR_CUDA, ERR_ALLOC, ERR_LIMIT = -1, -2, -3, -4, -5, -6
 NCOUNTS = 7
+TOPK_BY = {"abs": 0, "signed": 1}
+TOPK_MAX = 1024
 KERNEL_TILED, KERNEL_NAIVE = 0, 1
 PERSPECTIVE = {"global": 0, "local": 1, "complete": 2}
 ALTERNATIVE = {"two.sided": 0, "less": 1, "greater": 2}
@@ -36,7 +38,7 @@ EXPORTS = [
     "icikt_all_pairs_csc", "icikt_all_pairs_multi_csc", "icikt_pair_list_csc", "icikt_matrices_csc",
     "icikt_matrices_multi_csc", "icikt_pairwise_completeness_csc",
     "icikt_all_pairs_edges", "icikt_all_pairs_edges_csc", "icikt_edges_count", "icikt_edges_copy",
-    "icikt_edges_free",
+    "icikt_edges_free", "icikt_all_pairs_topk", "icikt_all_pairs_topk_csc",
 ]
 NSTATUS = 10
 
@@ -170,6 +172,12 @@ def load():
     L.icikt_edges_copy.restype = ctypes.c_int
     L.icikt_edges_free.argtypes = [vp]
     L.icikt_edges_free.restype = None
+    L.icikt_all_pairs_topk.argtypes = [_dp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, _dp, ctypes.c_int32,
+                                       ctypes.POINTER(Opts), ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _ip, _ip,
+                                       _dp, _dp, _dp, _dp, _dp, _dp, ctypes.POINTER(Timings)]
+    L.icikt_all_pairs_topk.restype = ctypes.c_int
+    L.icikt_all_pairs_topk_csc.argtypes = csc + L.icikt_all_pairs_topk.argtypes[4:]
+    L.icikt_all_pairs_topk_csc.restype = ctypes.c_int
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -367,6 +375,37 @@ def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=T
         check(L.icikt_edges_copy(h, _ptr(out["i"]), _ptr(out["j"]), *(_ptr(out[k]) for k in EDGE_NAMES)))
     finally:
         L.icikt_edges_free(h)
+    out.update(max_taumax=mx.value, timings=t.as_dict())
+    return out
+
+
+def run_topk(data, global_na=(), k=10, by="abs", scale_max=True, **opt_kw):
+    """icikt_all_pairs_topk: every column's k best partners over all pairs, selected on the device.
+
+    The candidates of column c are the columns d != c whose pair is not degenerate, ranked by abs(raw) (by="abs")
+    or raw (by="signed") descending, then d ascending; column c keeps its first min(k, #candidates), best first.
+    Every field is bit for bit run_pairs' for that pair, cor = raw / max_taumax if scale_max else raw.  data may be
+    a scipy.sparse matrix (-> icikt_all_pairs_topk_csc).  Returns a dict with index (C, k) int32 (-1 where
+    unused), cor, raw, pvalue, taumax, completeness (C, k) float64 (NaN where unused), n_neighbors (C,) int32,
+    max_taumax and timings."""
+    if by not in TOPK_BY:
+        raise ValueError(f"by must be one of {sorted(TOPK_BY)}")
+    L = load()
+    lead, sfx, n, C, keep_alive = _matrix_args(data)
+    o = make_opts(**opt_kw)
+    k = int(k)
+    kk = k if 1 <= k <= TOPK_MAX else 0  # a k the library refuses gets no arrays
+    k = k if -2 ** 31 <= k < 2 ** 31 else 0  # and reaches it as a refused int32
+    out = dict(index=np.empty((C, kk), dtype=np.int32))
+    out.update((name, np.empty((C, kk), dtype=np.float64)) for name in EDGE_NAMES)
+    out["n_neighbors"] = np.empty(C, dtype=np.int32)
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(getattr(L, "icikt_all_pairs_topk" + sfx)(*lead, gp, ng, ctypes.byref(o), k, TOPK_BY[by],
+                                                   int(bool(scale_max)), _ptr(out["index"]), _ptr(out["n_neighbors"]),
+                                                   *(_ptr(out[name]) for name in EDGE_NAMES), ctypes.byref(mx),
+                                                   ctypes.byref(t)))
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 

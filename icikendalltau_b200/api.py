@@ -364,6 +364,42 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     return out
 
 
+def ici_kendalltau_topk(data_matrix, k, by="abs", global_na=(np.nan, np.inf, 0), perspective="global",
+                        scale_max=True, alternative="two.sided", continuity=False, colnames=None, device=0):
+    """Every sample's k most correlated partners (a kNN table), over all pairs of a features x samples matrix.
+
+    The candidates of sample c are the samples d != c whose pair is not degenerate, ranked by abs(raw) (by="abs")
+    or raw (by="signed") descending, then by column position; c keeps its first min(k, #candidates), best first.
+    The selection runs on one GPU window by window (_lib.run_topk), so neither the result nor the device memory
+    grows with the number of pairs; degenerate pairs raise no warning.  Values are those of ici_kendalltau for the
+    same pair, cor = raw / max(taumax over all pairs) if scale_max else raw.
+
+    Returns a dict of (C, k) arrays `index` (int32, -1 where unused), `neighbors` (column names, None where
+    unused), `cor`, `raw`, `pvalue`, `taumax`, `completeness` (NaN where unused), plus `n_neighbors` (C,),
+    `max_taumax`, `run_time` and `names`.
+    """
+    if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.TOPK_MAX:
+        raise ValueError(f"`k` must be an integer in [1, {_lib.TOPK_MAX}], got {k!r}")
+    if by not in _lib.TOPK_BY:
+        raise ValueError(f"`by` must be 'abs' or 'signed', got {by!r}")
+    data, names = _colnames_of(data_matrix, colnames, "data_matrix")
+    global_na = [float(v) for v in global_na]
+    log.info("Running correlations ...")
+    t1 = time.perf_counter()
+    r = _lib.run_topk(data, global_na, int(k), by, scale_max, perspective=perspective, alternative=alternative,
+                      continuity=continuity, device=device)
+    run_time = time.perf_counter() - t1
+    nm = np.empty(len(names) + 1, dtype=object)  # the last entry, None, is what index -1 picks
+    for c, v in enumerate(names):
+        nm[c] = v
+    out = {key: r[key] for key in ("index", "cor", "raw", "pvalue", "taumax", "completeness", "n_neighbors",
+                                   "max_taumax")}
+    out["neighbors"] = nm[r["index"]]
+    out["run_time"] = run_time
+    out["names"] = names
+    return out
+
+
 _NA_METHODS = ("all.obs", "complete.obs", "pairwise.complete.obs", "everything", "na.or.complete")
 
 

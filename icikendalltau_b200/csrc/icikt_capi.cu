@@ -19,6 +19,7 @@
 #include "../../include/icikt_b200.h"
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
+#include "icikt_topk.cuh"
 
 using namespace icikt;
 
@@ -255,6 +256,14 @@ struct icikt_plan {
   unsigned long long* d_etotal = nullptr;  // [2]
   unsigned long long* h_estat = nullptr;   // pinned [2][2]: rows kept, max taumax bits so far
   cudaEvent_t eev[2][6]{};                 // per buffer: units up start/end, K2 start, K2 end, K3 end, selection end
+  // Top-k all-pairs call (icikt_all_pairs_topk), on the same window walk: per-column candidate counts, the
+  // candidates of one window, and the lists of up to topk_cap entries per column
+  uint32_t* d_tcount = nullptr;
+  uint2* d_tcand = nullptr;    // [2 W]
+  TopkCol* d_tcol = nullptr;   // [C]
+  int32_t* d_tidx = nullptr;   // [C k]
+  double* d_tlist = nullptr;   // 4 x [C k]: raw, pvalue, taumax, completeness
+  int topk_cap = 0;
 
   cudaEvent_t ev[9]{};
   icikt_timings tm{};
@@ -319,6 +328,11 @@ void free_plan(icikt_plan* p) {
   cudaFree(p->d_etile);
   cudaFree(p->d_etotal);
   if (p->h_estat) cudaFreeHost(p->h_estat);
+  cudaFree(p->d_tcount);
+  cudaFree(p->d_tcand);
+  cudaFree(p->d_tcol);
+  cudaFree(p->d_tidx);
+  cudaFree(p->d_tlist);
   for (auto& e : p->ev)
     if (e) cudaEventDestroy(e);
   for (auto& e : p->sync_ev)
@@ -1639,8 +1653,9 @@ struct icikt_edges {
   std::vector<double> cor;
 };
 
-// Pairs per window of the filtered call (ICIKT_EDGE_WINDOW, at most 2^30).  The default 2^26 keeps the window's
-// buffers near 10 GB: the plan's pair buffers (68 B per pair) and the two selected-row buffers (40 B each).
+// Pairs per window of the filtered calls, edges and top-k (ICIKT_EDGE_WINDOW, at most 2^30).  The default 2^26
+// keeps the window's buffers near 10 GB: the plan's pair buffers (68 B per pair) and the edge call's two
+// selected-row buffers (40 B each) or the top-k call's candidates (16 B).
 static int64_t edge_window() {
   const char* e = std::getenv("ICIKT_EDGE_WINDOW");
   const long long v = e ? std::atoll(e) : 0;
@@ -1653,13 +1668,9 @@ static double max_of_bits(unsigned long long bits) {
   return bits ? v : std::nan("");
 }
 
-// The argument checks of the filtered call, on the host before any device is touched.
-static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                           const icikt_opts& o, const icikt_edge_filter* f, icikt_edges** out) {
-  if (!out) return fail(ICIKT_ERR_BAD_ARG, "out is NULL");
-  *out = nullptr;
-  if (!f) return fail(ICIKT_ERR_BAD_ARG, "filter is NULL");
-  if (f->max_edges < 0) return fail(ICIKT_ERR_BAD_ARG, "max_edges must be >= 0 (0: no limit)");
+// The argument checks the filtered calls share, on the host before any device is touched.
+static int check_window_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na,
+                             int32_t n_global_na, const icikt_opts& o) {
   if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
   if (!s.csc() && (!s.data || s.ld < n)) return fail(ICIKT_ERR_BAD_ARG, "data must not be NULL and ld >= n");
   if (n > tiled_max_n()) return fail(ICIKT_ERR_TOO_LONG, "n exceeds icikt_max_n()");
@@ -1674,6 +1685,25 @@ static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const do
   return ICIKT_OK;
 }
 
+static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                           const icikt_opts& o, const icikt_edge_filter* f, icikt_edges** out) {
+  if (!out) return fail(ICIKT_ERR_BAD_ARG, "out is NULL");
+  *out = nullptr;
+  if (!f) return fail(ICIKT_ERR_BAD_ARG, "filter is NULL");
+  if (f->max_edges < 0) return fail(ICIKT_ERR_BAD_ARG, "max_edges must be >= 0 (0: no limit)");
+  return check_window_args(s, n, C, global_na, n_global_na, o);
+}
+
+static int check_topk_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                           const icikt_opts& o, int32_t k, int32_t by, const int32_t* index) {
+  if (k < 1 || k > ICIKT_TOPK_MAX) return fail(ICIKT_ERR_BAD_ARG, "k must be in [1, ICIKT_TOPK_MAX]");
+  if (by != ICIKT_TOPK_ABS && by != ICIKT_TOPK_SIGNED)
+    return fail(ICIKT_ERR_BAD_ARG, "by must be ICIKT_TOPK_ABS or ICIKT_TOPK_SIGNED");
+  if (!index) return fail(ICIKT_ERR_BAD_ARG, "index is NULL");
+  if (o.include_diag) return fail(ICIKT_ERR_BAD_ARG, "the top-k call ranks partners d != c: include_diag must be 0");
+  return check_window_args(s, n, C, global_na, n_global_na, o);
+}
+
 #define ECK(call)                                                                                              \
   do {                                                                                                         \
     cudaError_t e_ = (call);                                                                                   \
@@ -1682,20 +1712,48 @@ static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const do
                                              : cuda_fail(e_, #call);                                           \
   } while (0)
 
-// the selection's buffers for windows of W pairs (kept with the plan)
-static int ensure_edge_buffers(icikt_plan* p, int64_t W) {
+// the window walk's events, readbacks and staging chunks (kept with the plan)
+static int ensure_walk_buffers(icikt_plan* p) {
   if (p->d_etotal) return ICIKT_OK;
-  const int64_t tiles = (W + kEdgeTile - 1) / kEdgeTile;
   if (!p->copy_stream) ECK(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
-  ECK(dmalloc(&p->d_emask, (size_t)tiles * (kEdgeTile / 32)));
-  ECK(dmalloc(&p->d_etile, (size_t)tiles));
-  for (int b = 0; b < 2; ++b) {
-    ECK(dmalloc(&p->d_erows[b], (size_t)W));
+  for (int b = 0; b < 2; ++b)
     for (auto& e : p->eev[b]) ECK(cudaEventCreate(&e));
-  }
   ECK(cudaMallocHost(reinterpret_cast<void**>(&p->h_estat), 4 * sizeof(unsigned long long)));
   ECK(dmalloc(&p->d_etotal, 2));
   return ensure_stage(p);
+}
+
+// the edge selection's buffers for windows of W pairs (kept with the plan)
+static int ensure_edge_buffers(icikt_plan* p, int64_t W) {
+  const int rc = ensure_walk_buffers(p);
+  if (rc != ICIKT_OK || p->d_erows[1]) return rc;
+  const int64_t tiles = (W + kEdgeTile - 1) / kEdgeTile;
+  ECK(dmalloc(&p->d_emask, (size_t)tiles * (kEdgeTile / 32)));
+  ECK(dmalloc(&p->d_etile, (size_t)tiles));
+  for (int b = 0; b < 2; ++b) ECK(dmalloc(&p->d_erows[b], (size_t)W));
+  return ICIKT_OK;
+}
+
+// the top-k selection's buffers: candidates of a window of W pairs, and lists of k entries per column
+static int ensure_topk_buffers(icikt_plan* p, int64_t W, int k) {
+  const int rc = ensure_walk_buffers(p);
+  if (rc != ICIKT_OK) return rc;
+  if (!p->d_tcol) {
+    ECK(dmalloc(&p->d_tcount, (size_t)p->C));
+    ECK(dmalloc(&p->d_tcand, 2 * (size_t)W));
+    ECK(dmalloc(&p->d_tcol, (size_t)p->C));
+  }
+  if (k > p->topk_cap) {
+    cudaFree(p->d_tidx);
+    cudaFree(p->d_tlist);
+    p->d_tidx = nullptr;
+    p->d_tlist = nullptr;
+    p->topk_cap = 0;
+    ECK(dmalloc(&p->d_tidx, (size_t)p->C * k));
+    ECK(dmalloc(&p->d_tlist, 4 * (size_t)p->C * k));
+    p->topk_cap = k;
+  }
+  return ICIKT_OK;
 }
 
 // room for `need` units in both window unit buffers (device and pinned host)
@@ -1718,27 +1776,28 @@ static int ensure_window_units(icikt_plan* p, size_t need) {
   return ICIKT_OK;
 }
 
-// The filtered call on a plan whose pair buffers hold W pairs: upload and K1 once, then the pair order in windows
-// of W.  Window w is enqueued (units, K2, K3, selection, the readback of its row count and of the maximum so far)
-// before the host waits for window w - 1, copies its rows out on the copy stream and re-trims the rows it holds
-// against the new maximum; d_maxbits is not reset between windows, so K3's atomicMax leaves that maximum.
-static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
-                        const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
-                        icikt_timings* timings) {
-  int rc = ensure_edge_buffers(p, W);
-  if (rc == ICIKT_OK) rc = upload_columns(p, s, 0, p->C);
+// what the window walk adds up: event times, launches, and the maximum taumax so far (bits)
+struct WalkTotals {
+  float up_ms = 0.f, pairs_ms = 0.f, epi_ms = 0.f;
+  int launches = 0;
+  unsigned long long bits = 0;
+};
+
+// The window walk of the filtered calls, on a plan whose pair buffers hold W pairs: upload and K1 once, then the
+// pair order in windows of W.  Window w is enqueued (units, K2, K3, `select`, the readback of the maximum so
+// far) before the host waits for window w - 1 and runs `collect` for it; d_maxbits is not reset between
+// windows, so K3's atomicMax leaves that maximum.  select(w, b, units, n_units, n_slots) enqueues the
+// selection of window w on p->stream (b: its buffer, 0 or 1); collect(w, b) runs once that has completed.
+template <class Select, class Collect>
+static int walk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
+                        int64_t ptot, int64_t W, WalkTotals& tot, Select&& select, Collect&& collect) {
+  int rc = upload_columns(p, s, 0, p->C);
   if (rc == ICIKT_OK) rc = plan_columns_impl(p, global_na, n_global_na, 0, p->C, true);
   if (rc != ICIKT_OK) return rc;
-  int launches = p->tm.n_launches;
+  tot.launches = p->tm.n_launches;
   CK(cudaMemsetAsync(p->d_maxbits, 0, sizeof(unsigned long long), p->stream));
-  const double t = f.min_abs_cor;
-  const bool scale = f.scale_max != 0;
-  const bool retrim = scale && t == t;
   const int64_t nwin = (ptot + W - 1) / W, ptri = tri_pairs(p->C), slots = (int64_t)p->n_sm * 2;
   std::vector<PairUnit> U;
-  std::vector<EdgeRow>& rows = res->rows;
-  float up_ms = 0.f, pairs_ms = 0.f, epi_ms = 0.f, d2h_ms = 0.f;
-  unsigned long long bits = 0, trimmed_bits = 0;
 
   auto enqueue = [&](int64_t w) -> int {
     const int b = (int)(w & 1);
@@ -1757,12 +1816,75 @@ static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* glob
     CK(cudaEventRecord(e[0], p->stream));
     CK(cudaMemcpyAsync(p->d_wunits[b], p->h_wunits[b], sizeof(PairUnit) * U.size(), cudaMemcpyHostToDevice, p->stream));
     CK(cudaEventRecord(e[1], p->stream));
-    r = launch_pair_group(p, p->d_wunits[b], 0, (int64_t)U.size(), max_unit, e[2], e[3], e[4], &launches);
+    r = launch_pair_group(p, p->d_wunits[b], 0, (int64_t)U.size(), max_unit, e[2], e[3], e[4], &tot.launches);
     if (r != ICIKT_OK) return r;
+    r = select(w, b, p->d_wunits[b], (int64_t)U.size(), hi - lo);
+    if (r != ICIKT_OK) return r;
+    CK(cudaMemcpyAsync(p->h_estat + 2 * b + 1, p->d_maxbits, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaEventRecord(e[5], p->stream));
+    return ICIKT_OK;
+  };
+
+  auto wait = [&](int64_t w) -> int {
+    const int b = (int)(w & 1);
+    cudaEvent_t* e = p->eev[b];
+    CK(cudaEventSynchronize(e[5]));
+    tot.bits = p->h_estat[2 * b + 1];
+    tot.up_ms += ev_ms(e[0], e[1]);
+    tot.pairs_ms += ev_ms(e[2], e[3]);
+    tot.epi_ms += ev_ms(e[3], e[5]);
+    return collect(w, b);
+  };
+
+  for (int64_t w = 0; w <= nwin; ++w) {
+    if (w < nwin && (rc = enqueue(w)) != ICIKT_OK) return rc;
+    if (w > 0 && (rc = wait(w - 1)) != ICIKT_OK) return rc;
+  }
+  return ICIKT_OK;
+}
+
+// the end of a walk: both streams drained, then the timings (d2h_ms: the caller's copies out)
+static int finish_walk(icikt_plan* p, const WalkTotals& tot, float d2h_ms, icikt_timings* timings) {
+  CK(cudaEventRecord(p->ev[4], p->copy_stream));
+  CK(cudaStreamWaitEvent(p->stream, p->ev[4], 0));
+  CK(cudaEventRecord(p->ev[5], p->stream));
+  CK(cudaEventSynchronize(p->ev[5]));
+  if (timings) {
+    std::memset(timings, 0, sizeof(*timings));
+    timings->h2d_ms = ev_ms(p->ev[0], p->ev[1]) + tot.up_ms;
+    timings->columns_ms = ev_ms(p->ev[2], p->ev[3]);
+    timings->pairs_ms = tot.pairs_ms;
+    timings->epilogue_ms = tot.epi_ms;
+    timings->d2h_ms = d2h_ms;
+    timings->total_ms = ev_ms(p->ev[0], p->ev[5]);
+    timings->n_launches = tot.launches;
+    cudaGetLastError();
+  }
+  return ICIKT_OK;
+}
+
+// The filtered call: per window, the edge selection and the readback of its row count; once the host has waited
+// for a window, its rows are copied out on the copy stream and the rows held are re-trimmed against the new
+// maximum.
+static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
+                        const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
+                        icikt_timings* timings) {
+  int rc = ensure_edge_buffers(p, W);
+  if (rc != ICIKT_OK) return rc;
+  const double t = f.min_abs_cor;
+  const bool scale = f.scale_max != 0;
+  const bool retrim = scale && t == t;
+  const int64_t nwin = (ptot + W - 1) / W;
+  std::vector<EdgeRow>& rows = res->rows;
+  WalkTotals tot;
+  float d2h_ms = 0.f;
+  unsigned long long trimmed_bits = 0;
+
+  auto select = [&](int64_t, int b, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
     EdgeSelect es;
-    es.units = p->d_wunits[b];
-    es.n_units = (int64_t)U.size();
-    es.n_slots = hi - lo;
+    es.units = units;
+    es.n_units = n_units;
+    es.n_slots = n_slots;
     es.tau = p->d_tau;
     es.pvalue = p->d_p;
     es.taumax = p->d_tm;
@@ -1778,22 +1900,14 @@ static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* glob
     es.rows = p->d_erows[b];
     const int l = launch_edge_select(es, p->stream);
     if (l < 0) return launch_fail("edge selection kernels");
-    launches += l;
+    tot.launches += l;
     CK(cudaMemcpyAsync(p->h_estat + 2 * b, p->d_etotal + b, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
-    CK(cudaMemcpyAsync(p->h_estat + 2 * b + 1, p->d_maxbits, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
-    CK(cudaEventRecord(e[5], p->stream));
     return ICIKT_OK;
   };
 
-  auto collect = [&](int64_t w) -> int {
-    const int b = (int)(w & 1);
-    cudaEvent_t* e = p->eev[b];
-    CK(cudaEventSynchronize(e[5]));
+  auto collect = [&](int64_t w, int b) -> int {
     const unsigned long long cnt = p->h_estat[2 * b];
-    bits = p->h_estat[2 * b + 1];
-    up_ms += ev_ms(e[0], e[1]);
-    pairs_ms += ev_ms(e[2], e[3]);
-    epi_ms += ev_ms(e[3], e[5]);
+    const unsigned long long bits = tot.bits;
     if (cnt) {
       const size_t old = rows.size();
       try {
@@ -1821,12 +1935,10 @@ static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* glob
     return ICIKT_OK;
   };
 
-  for (int64_t w = 0; w <= nwin; ++w) {
-    if (w < nwin && (rc = enqueue(w)) != ICIKT_OK) return rc;
-    if (w > 0 && (rc = collect(w - 1)) != ICIKT_OK) return rc;
-  }
+  rc = walk_windows(p, s, global_na, n_global_na, ptot, W, tot, select, collect);
+  if (rc != ICIKT_OK) return rc;
   // the exact predicate with the final maximum
-  const double M = max_of_bits(bits);
+  const double M = max_of_bits(tot.bits);
   if (scale && t == t)
     rows.erase(std::remove_if(rows.begin(), rows.end(), [&](const EdgeRow& r) { return !edge_keep_final(r.raw, t, true, M); }),
                rows.end());
@@ -1835,25 +1947,135 @@ static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* glob
                                      std::to_string(rows.size()) + ")");
   res->cor.resize(rows.size());
   for (size_t k = 0; k < rows.size(); ++k) res->cor[k] = scale ? rows[k].raw / M : rows[k].raw;
-  CK(cudaEventRecord(p->ev[4], p->copy_stream));
-  CK(cudaStreamWaitEvent(p->stream, p->ev[4], 0));
-  CK(cudaEventRecord(p->ev[5], p->stream));
-  CK(cudaEventSynchronize(p->ev[5]));
+  rc = finish_walk(p, tot, d2h_ms, timings);
+  if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = M;
-  if (timings) {
-    std::memset(timings, 0, sizeof(*timings));
-    timings->h2d_ms = ev_ms(p->ev[0], p->ev[1]) + up_ms;
-    timings->columns_ms = ev_ms(p->ev[2], p->ev[3]);
-    timings->pairs_ms = pairs_ms;
-    timings->epilogue_ms = epi_ms;
-    timings->d2h_ms = d2h_ms;
-    timings->total_ms = ev_ms(p->ev[0], p->ev[5]);
-    timings->n_launches = launches;
-    cudaGetLastError();
+  return ICIKT_OK;
+}
+
+// The top-k call: per window, the top-k selection merges the window's candidates into the lists on the device;
+// nothing comes back until the last window, then the lists are copied out once and cor is formed with the
+// final maximum.
+static_assert(kTopkMax == ICIKT_TOPK_MAX, "the merge kernel holds one list entry per thread");
+struct TopkOut {
+  int32_t *index, *n_neighbors;
+  double *cor, *raw, *pvalue, *taumax, *completeness;
+};
+
+static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na, int k,
+                        int by, bool scale, int64_t ptot, int64_t W, const TopkOut& out, double* max_taumax,
+                        icikt_timings* timings) {
+  int rc = ensure_topk_buffers(p, W, k);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t C = p->C, ck = C * k;
+  CK(cudaMemsetAsync(p->d_tcol, 0, sizeof(TopkCol) * (size_t)C, p->stream));
+  double* d_raw = p->d_tlist;
+  double* d_field[3] = {p->d_tlist + ck, p->d_tlist + 2 * ck, p->d_tlist + 3 * ck};
+  WalkTotals tot;
+
+  auto select = [&](int64_t, int b, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
+    TopkSelect ts;
+    ts.units = units;
+    ts.n_units = n_units;
+    ts.n_slots = n_slots;
+    ts.tau = p->d_tau;
+    ts.pvalue = p->d_p;
+    ts.taumax = p->d_tm;
+    ts.completeness = p->d_comp;
+    ts.status = p->d_status;
+    ts.C = C;
+    ts.k = k;
+    ts.by = by;
+    ts.col_count = p->d_tcount;
+    ts.total = p->d_etotal + b;
+    ts.cand = p->d_tcand;
+    ts.col = p->d_tcol;
+    ts.idx = p->d_tidx;
+    ts.raw = d_raw;
+    ts.pv = d_field[0];
+    ts.tm = d_field[1];
+    ts.comp = d_field[2];
+    const int l = launch_topk_select(ts, p->stream);
+    if (l < 0) return launch_fail("top-k selection kernels");
+    tot.launches += l;
+    return ICIKT_OK;
+  };
+
+  rc = walk_windows(p, s, global_na, n_global_na, ptot, W, tot, select, [](int64_t, int) { return ICIKT_OK; });
+  if (rc != ICIKT_OK) return rc;
+  // the lists, once
+  std::vector<TopkCol> col;
+  std::vector<double> raw_own;
+  double* raw = out.raw;
+  try {
+    col.resize((size_t)C);
+    if (!raw && out.cor) {
+      raw_own.resize((size_t)ck);
+      raw = raw_own.data();
+    }
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
   }
+  CK(cudaEventRecord(p->ev[6], p->stream));
+  rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)C, p->stream);
+  if (rc == ICIKT_OK) rc = staged_copy_out(p, out.index, p->d_tidx, sizeof(int32_t) * (size_t)ck, p->stream);
+  if (rc == ICIKT_OK && raw) rc = staged_copy_out(p, raw, d_raw, sizeof(double) * (size_t)ck, p->stream);
+  double* host_field[3] = {out.pvalue, out.taumax, out.completeness};
+  for (int f = 0; f < 3 && rc == ICIKT_OK; ++f)
+    if (host_field[f]) rc = staged_copy_out(p, host_field[f], d_field[f], sizeof(double) * (size_t)ck, p->stream);
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[7], p->stream));
+  CK(cudaEventSynchronize(p->ev[7]));
+  const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
+  const double M = max_of_bits(tot.bits);
+  const double qnan = std::nan("");
+  for (int64_t c = 0; c < C; ++c) {
+    const int64_t held = col[(size_t)c].n, base = c * k;
+    if (out.n_neighbors) out.n_neighbors[c] = (int32_t)held;
+    if (out.cor)
+      for (int64_t r = 0; r < held; ++r) out.cor[base + r] = scale ? raw[base + r] / M : raw[base + r];
+    for (int64_t r = held; r < k; ++r) {
+      out.index[base + r] = -1;
+      for (double* a : {out.cor, out.raw, out.pvalue, out.taumax, out.completeness})
+        if (a) a[base + r] = qnan;
+    }
+  }
+  rc = finish_walk(p, tot, d2h_ms, timings);
+  if (rc != ICIKT_OK) return rc;
+  if (max_taumax) *max_taumax = M;
   return ICIKT_OK;
 }
 #undef ECK
+
+// The plan of the filtered calls (cached in g_cached_edges; the caller holds g_cache_mu): pair buffers of one
+// window of W pairs.
+static int window_plan(int64_t n, int64_t C, int64_t W, const icikt_opts& o, icikt_plan** out) {
+  icikt_plan* p = g_cached_edges;
+  if (p && p->n == n && p->C == C && p->P == W && p->opts.device == o.device && p->opts.include_diag == o.include_diag) {
+    p->opts.perspective = o.perspective;
+    p->opts.alternative = o.alternative;
+    p->opts.continuity = o.continuity;
+    p->opts.na_inf = o.na_inf;
+  } else {
+    if (p) icikt_plan_destroy(p);
+    g_cached_edges = nullptr;
+    icikt_opts po = o;
+    po.pair_hi = W;  // the plan's pair buffers: one window
+    const int rc = plan_create_impl(&p, n, C, nullptr, nullptr, 0, &po, false);
+    if (rc != ICIKT_OK) return rc;
+    g_cached_edges = p;
+  }
+  *out = p;
+  return ICIKT_OK;
+}
+
+// after a failed call: the cached plan goes, keeping the call's error message
+static void drop_window_plan() {
+  const std::string keep = g_err;
+  icikt_plan_destroy(g_cached_edges);  // waits for whatever the failed call left in flight
+  g_cached_edges = nullptr;
+  g_err = keep;
+}
 
 static int all_pairs_edges(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
                            const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
@@ -1875,35 +2097,47 @@ static int all_pairs_edges(const ColumnSource& s, int64_t n, int64_t C, const do
   }
   const int64_t W = std::min(edge_window(), ptot);
   std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = g_cached_edges;
-  if (p && p->n == n && p->C == C && p->P == W && p->opts.device == o.device && p->opts.include_diag == o.include_diag) {
-    p->opts.perspective = o.perspective;
-    p->opts.alternative = o.alternative;
-    p->opts.continuity = o.continuity;
-    p->opts.na_inf = o.na_inf;
-  } else {
-    if (p) icikt_plan_destroy(p);
-    g_cached_edges = nullptr;
-    icikt_opts po = o;
-    po.pair_hi = W;  // the plan's pair buffers: one window
-    rc = plan_create_impl(&p, n, C, nullptr, nullptr, 0, &po, false);
-    if (rc != ICIKT_OK) {
-      delete res;
-      return rc;
-    }
-    g_cached_edges = p;
-  }
-  rc = edge_windows(p, s, global_na, n_global_na, *filter, ptot, W, res, max_taumax, timings);
+  icikt_plan* p = nullptr;
+  rc = window_plan(n, C, W, o, &p);
+  if (rc == ICIKT_OK) rc = edge_windows(p, s, global_na, n_global_na, *filter, ptot, W, res, max_taumax, timings);
   if (rc != ICIKT_OK) {
-    const std::string keep = g_err;
-    icikt_plan_destroy(g_cached_edges);  // waits for whatever the failed call left in flight
-    g_cached_edges = nullptr;
+    drop_window_plan();
     delete res;
-    g_err = keep;
     return rc;
   }
   *out = res;
   return ICIKT_OK;
+}
+
+static int all_pairs_topk(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                          const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max, const TopkOut& out,
+                          double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  int rc = check_topk_args(s, n, C, global_na, n_global_na, o, k, by, out.index);
+  if (rc != ICIKT_OK) return rc;
+  rc = select_device(o.device);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t ptot = tri_pairs(C);
+  if (ptot == 0) {  // one column: no candidate
+    for (int32_t r = 0; r < k; ++r) {
+      out.index[r] = -1;
+      for (double* a : {out.cor, out.raw, out.pvalue, out.taumax, out.completeness})
+        if (a) a[r] = std::nan("");
+    }
+    if (out.n_neighbors) out.n_neighbors[0] = 0;
+    if (max_taumax) *max_taumax = std::nan("");
+    if (timings) std::memset(timings, 0, sizeof(*timings));
+    return ICIKT_OK;
+  }
+  const int64_t W = std::min(edge_window(), ptot);
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  icikt_plan* p = nullptr;
+  rc = window_plan(n, C, W, o, &p);
+  if (rc == ICIKT_OK)
+    rc = topk_windows(p, s, global_na, n_global_na, k, by, scale_max != 0, ptot, W, out, max_taumax, timings);
+  if (rc != ICIKT_OK) drop_window_plan();
+  return rc;
 }
 
 extern "C" {
@@ -1945,6 +2179,25 @@ int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, 
 }
 
 void icikt_edges_free(icikt_edges* e) { delete e; }
+
+int icikt_all_pairs_topk(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                         int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                         int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
+                         double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
+  return all_pairs_topk(dense_source(data, ld), n, C, global_na, n_global_na, opts, k, by, scale_max,
+                        TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
+}
+
+int icikt_all_pairs_topk_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                             int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                             int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
+                             double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                             double* max_taumax, icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return all_pairs_topk(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, k, by, scale_max,
+                        TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
+}
 
 }  // extern "C"
 

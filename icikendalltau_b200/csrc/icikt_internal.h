@@ -224,6 +224,33 @@ struct EdgeSelect {
 };
 int launch_edge_select(const EdgeSelect& s, cudaStream_t stream);
 
+// The selection of the top-k all-pairs call (icikt_select.cu), per window: a count pass tests both candidates of
+// every valid slot (column i gets partner j, column j gets i) against the column's k-th entry, one CTA scans the
+// column counts into bucket offsets, a scatter pass fills the buckets, and one CTA per column merges its bucket
+// into the column's sorted list (order of icikt_topk.cuh), gathering the new entries' fields from the window.
+constexpr int kTopkMax = 1024;  // ICIKT_TOPK_MAX
+struct TopkCol {
+  unsigned long long key;  // the k-th entry's key and partner, once n == k
+  int32_t idx;
+  int32_t n;               // entries held
+};
+struct TopkSelect {
+  const PairUnit* units;  // device, the window's units (slots relative to the window)
+  int64_t n_units;
+  int64_t n_slots;        // pairs in the window
+  const double *tau, *pvalue, *taumax, *completeness;
+  const int32_t* status;
+  int64_t C;
+  int k, by;
+  uint32_t* col_count;    // device [C]: candidates per column, then the end of every column's bucket
+  unsigned long long* total;  // device, candidates in the window
+  uint2* cand;            // device [2 n_slots]: (window slot, partner)
+  TopkCol* col;           // device [C], zero before the first window
+  int32_t* idx;           // device [C k]: the sorted lists
+  double *raw, *pv, *tm, *comp;  // device [C k]
+};
+int launch_topk_select(const TopkSelect& s, cudaStream_t stream);
+
 int launch_pnorm(const double* d_z, int64_t n, int lower, double* d_out, cudaStream_t stream);
 
 int64_t tiled_max_n();

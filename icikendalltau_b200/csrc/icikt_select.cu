@@ -8,8 +8,11 @@
 //     bits below it.  Tiles without a kept slot stop after reading their 32 words.
 // HBM-bound: the count pass reads the status and, only for a bound that is given, raw (8 B) and the p-value
 // (8 B); the scatter pass reads 1/8 B of mask per slot and the fields of the kept slots.
+// The selection of the top-k call (icikt_all_pairs_topk) follows the edge kernels: per-column buckets of the
+// candidates that beat a column's k-th entry, merged into the column's sorted list (see launch_topk_select).
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
+#include "icikt_topk.cuh"
 
 namespace icikt {
 
@@ -153,7 +156,176 @@ __global__ void __launch_bounds__(kSelThreads) edge_scatter_kernel(const EdgeSel
   }
 }
 
+// Top-k: the count pass (kScatter false) and the scatter pass (true) of one tile of kEdgeTile slots.  Both make
+// the same decisions, against the thresholds the previous window's merge left.  A unit's pairs share column i,
+// so its candidates for i are counted with one atomic per warp and column.
+__device__ __forceinline__ bool topk_takes(const TopkCol& t, int k, unsigned long long key, int32_t partner) {
+  return t.n < k || topk_before(key, partner, t.key, t.idx);
+}
+
+template <bool kScatter>
+__global__ void __launch_bounds__(kSelThreads) topk_bucket_kernel(const TopkSelect s) {
+  __shared__ long long unit_range[2];
+  const long long tile = blockIdx.x;
+  const int lane = threadIdx.x & 31;
+  if (threadIdx.x < 2) {
+    const long long first_slot = tile * kEdgeTile;
+    const long long last_slot = min((long long)s.n_slots, first_slot + kEdgeTile) - 1;
+    unit_range[threadIdx.x] = unit_of(s.units, 0, s.n_units, threadIdx.x ? last_slot : first_slot);
+  }
+  __syncthreads();
+  const long long ua = unit_range[0], ub = unit_range[1] + 1;
+  for (int r = 0; r < kSelRounds; ++r) {
+    const long long slot = tile * kEdgeTile + r * kSelThreads + threadIdx.x;
+    int32_t i = -1, j = -1;
+    bool take_i = false, take_j = false;
+    if (slot < s.n_slots && s.status[slot] == 0) {
+      const PairUnit u = s.units[unit_of(s.units, ua, ub, slot)];
+      i = u.col;
+      j = u.j0 + (int32_t)(slot - u.slot0);
+      const unsigned long long key = topk_key(s.tau[slot], s.by);
+      take_i = topk_takes(s.col[i], s.k, key, j);
+      take_j = topk_takes(s.col[j], s.k, key, i);
+    }
+    const unsigned peers = __match_any_sync(FULL, take_i ? i : -1);
+    if (take_i) {
+      const int leader = __ffs(peers) - 1;
+      unsigned at = 0;
+      if (lane == leader) at = atomicAdd(&s.col_count[i], (unsigned)__popc(peers));
+      if (kScatter) {
+        at = __shfl_sync(peers, at, leader) + __popc(peers & ((1u << lane) - 1u));
+        s.cand[at] = make_uint2((unsigned)slot, (unsigned)j);
+      }
+    }
+    if (take_j) {
+      const unsigned at = atomicAdd(&s.col_count[j], 1u);
+      if (kScatter) s.cand[at] = make_uint2((unsigned)slot, (unsigned)i);
+    }
+  }
+}
+
+// One CTA per column: its bucket is taken in chunks that fill a shared array behind the list; candidates that
+// cannot beat the list's k-th entry are dropped, the rest are sorted with the list (bitonic) and the first k
+// kept.  Then every thread gathers one entry's fields, from the list or from the window, before any is written.
+constexpr int kMergeThreads = kTopkMax;
+constexpr int kMergeCap = 2 * kTopkMax;
+static_assert(kMergeCap - kTopkMax >= kMergeThreads, "a chunk holds at least one candidate per thread");
+
+__global__ void __launch_bounds__(kMergeThreads) topk_merge_kernel(const TopkSelect s) {
+  __shared__ unsigned long long key[kMergeCap];
+  __shared__ int32_t part[kMergeCap];
+  __shared__ int32_t src[kMergeCap];  // >= 0: window slot; < 0: -1 - position in the list
+  __shared__ int fill;
+  const long long c = blockIdx.x;
+  const uint32_t end = s.col_count[c], beg = c ? s.col_count[c - 1] : 0u;
+  if (end == beg) return;
+  const int k = s.k, tid = threadIdx.x;
+  const long long base = c * k;
+  int n = s.col[c].n;
+  if (tid < n) {
+    key[tid] = topk_key(s.raw[base + tid], s.by);
+    part[tid] = s.idx[base + tid];
+    src[tid] = -1 - tid;
+  }
+  for (uint32_t o = beg; o < end;) {
+    const uint32_t take = min(end - o, (uint32_t)(kMergeCap - n));
+    if (tid == 0) fill = n;
+    __syncthreads();
+    const bool full = n == k;
+    const unsigned long long tk = full ? key[k - 1] : 0ull;
+    const int32_t ti = full ? part[k - 1] : 0;
+    for (uint32_t q = tid; q < take; q += kMergeThreads) {
+      const uint2 e = s.cand[o + q];
+      const unsigned long long kk = topk_key(s.tau[e.x], s.by);
+      if (!full || topk_before(kk, (int32_t)e.y, tk, ti)) {
+        const int at = atomicAdd(&fill, 1);
+        key[at] = kk;
+        part[at] = (int32_t)e.y;
+        src[at] = (int32_t)e.x;
+      }
+    }
+    o += take;
+    __syncthreads();
+    const int m = fill;
+    __syncthreads();
+    if (m == n) continue;
+    int L = 2;
+    while (L < m) L <<= 1;
+    for (int q = m + tid; q < L; q += kMergeThreads) {  // padding that sorts last
+      key[q] = 0ull;
+      part[q] = 0x7fffffff;
+    }
+    __syncthreads();
+    for (int size = 2; size <= L; size <<= 1) {
+      for (int stride = size >> 1; stride > 0; stride >>= 1) {
+        for (int t = tid; t < L / 2; t += kMergeThreads) {
+          const int lo = 2 * t - (t & (stride - 1)), hi = lo + stride;
+          const bool up = (lo & size) == 0;
+          if (topk_before(key[hi], part[hi], key[lo], part[lo]) == up) {
+            const unsigned long long tk2 = key[lo];
+            key[lo] = key[hi];
+            key[hi] = tk2;
+            const int32_t tp = part[lo];
+            part[lo] = part[hi];
+            part[hi] = tp;
+            const int32_t ts = src[lo];
+            src[lo] = src[hi];
+            src[hi] = ts;
+          }
+        }
+        __syncthreads();
+      }
+    }
+    n = min(m, k);
+  }
+  double raw = 0.0, pv = 0.0, tm = 0.0, comp = 0.0;
+  if (tid < n) {
+    const int32_t from = src[tid];
+    if (from < 0) {
+      const long long q = base + (-1 - from);
+      raw = s.raw[q];
+      pv = s.pv[q];
+      tm = s.tm[q];
+      comp = s.comp[q];
+    } else {
+      raw = s.tau[from];
+      pv = s.pvalue[from];
+      tm = s.taumax[from];
+      comp = s.completeness[from];
+    }
+  }
+  __syncthreads();
+  if (tid < n) {
+    s.idx[base + tid] = part[tid];
+    s.raw[base + tid] = raw;
+    s.pv[base + tid] = pv;
+    s.tm[base + tid] = tm;
+    s.comp[base + tid] = comp;
+  }
+  if (tid == 0) {
+    TopkCol t;
+    t.n = n;
+    t.key = n == k ? key[k - 1] : 0ull;
+    t.idx = n == k ? part[k - 1] : 0;
+    s.col[c] = t;
+  }
+}
+
 }  // namespace
+
+int launch_topk_select(const TopkSelect& s, cudaStream_t stream) {
+  if (s.n_slots <= 0) return launch_status(0);
+  const long long tiles = (s.n_slots + kEdgeTile - 1) / kEdgeTile;
+  if (tiles > 0x7fffffffLL || s.C > 0x7fffffffLL || 2 * s.n_slots > 0xffffffffLL)
+    return launch_refused("top-k selection: window too large");
+  if (cudaMemsetAsync(s.col_count, 0, sizeof(uint32_t) * (size_t)s.C, stream) != cudaSuccess)
+    return launch_refused("top-k selection: clearing the column counts");
+  topk_bucket_kernel<false><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  edge_scan_kernel<<<1, 1024, 0, stream>>>(s.col_count, s.C, s.total);
+  topk_bucket_kernel<true><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  topk_merge_kernel<<<(unsigned)s.C, kMergeThreads, 0, stream>>>(s);
+  return launch_status(4);
+}
 
 int launch_edge_select(const EdgeSelect& s, cudaStream_t stream) {
   if (s.n_slots <= 0) {

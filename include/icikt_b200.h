@@ -275,6 +275,43 @@ int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, 
                      double* taumax, double* completeness);
 void icikt_edges_free(icikt_edges* e);
 
+/* ---- all pairs, each column's k most correlated partners (the kNN table of a wide matrix), selected on the
+ * device over the same windows of the pair order as the filtered call above (ICIKT_EDGE_WINDOW).  For column c
+ * the candidates are every d != c whose pair (min(c, d), max(c, d)) has status == 0; degenerate pairs are never
+ * candidates and raise no warning.  Candidates are ranked by a strict total order:
+ *
+ *   by = ICIKT_TOPK_ABS:    |raw| descending, then d ascending
+ *   by = ICIKT_TOPK_SIGNED:  raw  descending, then d ascending  (-0.0 equal to +0.0)
+ *
+ * and column c keeps the first min(k, #candidates) of them, best first.  The ranking is on raw, not on cor:
+ * two raws that differ keep their order even where they round to the same cor = raw / M.
+ * Outputs are caller-allocated C x k arrays, entry r of column c at c*k + r: index (required) the partner d;
+ * cor (scale_max ? raw / M : raw, M = max(taumax) over all computed pairs, the IEEE division of
+ * icikt_plan_download_matrices), raw, pvalue, taumax, completeness (each may be NULL) bit for bit what
+ * icikt_all_pairs returns for that pair.  Unused entries hold index -1 and a quiet NaN in every double;
+ * n_neighbors [C] (may be NULL) the entries kept.  k > C - 1 only pads; C == 1 pads everything and M is NaN.
+ * Device memory does not depend on P: the per-column tables, one window of pairs, its candidates (16 B per
+ * pair) and the lists (36 B per entry).
+ * Options: perspective global or local, alternative, continuity, na_inf, device.  Refused with
+ * ICIKT_ERR_BAD_ARG before any device is touched: k < 1 or k > ICIKT_TOPK_MAX, by not ABS or SIGNED, a NULL
+ * index, include_diag, pair_lo / pair_hi != 0, ICIKT_PERSPECTIVE_COMPLETE, ICIKT_KERNEL_NAIVE, want_counts.
+ * max_taumax (may be NULL) M or NaN.  timings (may be NULL): pairs_ms is the sum of K2 over the windows,
+ * epilogue_ms of K3 and the selection, d2h_ms the copy of the lists. */
+#define ICIKT_TOPK_ABS 0
+#define ICIKT_TOPK_SIGNED 1
+#define ICIKT_TOPK_MAX 1024
+
+int icikt_all_pairs_topk(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                         int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                         int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
+                         double* taumax, double* completeness, double* max_taumax, icikt_timings* timings);
+/* the same for a CSC matrix (see the sparse calls above) */
+int icikt_all_pairs_topk_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                             int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                             int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
+                             double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                             double* max_taumax, icikt_timings* timings);
+
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
  * pay the copies.  A plan is bound to one device and is not thread-safe.            */
