@@ -397,19 +397,32 @@ __host__ __device__ constexpr int count_pass_barriers(int L) { return 2 * (L > 4
 // partition keeps a leading block of them exactly where it is; no one-key ever precedes them, so they
 // add nothing to any count.  Threads whose whole range lies inside that block skip the sweeps of
 // every level (they only take part in the scans, with zero counts, and in the barriers).
-template <bool G>
+// TAIL (besides `lead`): only the first `len` keys are the sequence, the rest is all-ones padding
+// (2^L - 1); len = cap for a full sequence.  Padding is the largest key, so it is in the last non-empty class at every level and
+// the stable partition keeps it where it is; it never adds to a count.  Threads whose whole range
+// lies at or beyond `len` skip the sweeps of every level: they enter the scans with the class
+// counts of R padding keys (closed form) and add nothing; nobody reads their ranges.  The thread
+// that straddles `len` writes the padding of its own range before its first sweep.
+template <bool G, bool TAIL = false>
 __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<G>::ptr b, const int kk,
                                            const int nwarps, const int L, uint32_t* descA, uint32_t* descB,
                                            const int lane, const int warp, const PipeConst pc,
-                                           unsigned long long& acc64, const uint32_t lead = 0u) {
+                                           unsigned long long& acc64, const uint32_t lead = 0u,
+                                           const uint32_t len = 0u) {
   typedef Mem<G> M;
   const uint32_t tid = ((uint32_t)warp << 5) + (uint32_t)lane;
   const uint32_t R = (uint32_t)kk << 3;                // keys per thread range
   const uint32_t my_off = tid * (R << 1);              // bytes
   const uint32_t my_pos = tid * R;
   const uint32_t cap = ((uint32_t)nwarps << 5) * R;    // keys per buffer
-  const bool idle = my_pos + R <= lead;
-  if (idle && L > 4) {  // the block must read as zeros in the other buffer too (levels alternate)
+  const uint32_t padA = (1u << L) - 1u;
+  const bool tail = TAIL && my_pos >= len;
+  const bool idle = tail || my_pos + R <= lead;
+  if constexpr (TAIL) {
+    if (!idle)
+      for (uint32_t q = len; q < my_pos + R; ++q) M::st16(M::add(a, (int32_t)(q << 1)), padA);
+  }
+  if (idle && !tail && L > 4) {  // the block must read as zeros in the other buffer too (levels alternate)
     const typename M::ptr rb = M::add(b, (int32_t)my_off);
     for (int c = 0; c < kk; ++c) M::st128(M::add(rb, c << 4), 0u, 0u, 0u, 0u);
   }
@@ -435,7 +448,14 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     wm += chj[1] + 2u * chj[2] + 3u * chj[3];
     const LevelCounts lc = fold_counts(cl, ch, cb, wm);
     const uint32_t n1 = lc.n1, n2 = lc.n2, n3 = lc.n3;
-    const uint32_t A = n1 | (n2 << 16), B = n3;
+    uint32_t A = n1 | (n2 << 16), B = n3;
+    if constexpr (TAIL) {
+      if (tail) {  // R padding keys: class 3, or class 1 on the first level of an odd L (its top bit is 0)
+        const uint32_t pcl = (padA >> s) & 3u;
+        A = pcl == 1u ? R : 0u;
+        B = pcl == 3u ? R : 0u;
+      }
+    }
     uint32_t inclA = A, inclB = B;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {

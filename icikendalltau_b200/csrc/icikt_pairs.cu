@@ -291,7 +291,9 @@ struct PwSide {
 //   the counters also yields, from the other column's group-start table, everything needed to
 //   take the group's rows out of the pair: see PwSide.  `a_tbl` = missing rows of the other column.
 //   GT: the rank table is read from global memory instead of the staged copy.
-template <bool G, bool EMIT, bool PW, bool GT>
+//   CZ and skip0: the rows with the other column's lowest rank are counted (ties, mini[18]) but not
+//   written: the emitted sequence starts with the group's first nonzero rank (see compact_gather).
+template <bool G, bool EMIT, bool PW, bool GT, bool CZ = false>
 __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const int cap, const int keep,
                                                const int nrows, const int K,
                                                const uint16_t* __restrict__ rows,
@@ -302,8 +304,10 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
                                                const int nwarps, const uint16_t* __restrict__ gstart,
                                                const int a_tbl, PwSide& pw, const bool try_bits = false,
                                                const uint32_t* __restrict__ grp_bits = nullptr,
-                                               const uint32_t* nab_other = nullptr, const int nwords = 0) {
+                                               const uint32_t* nab_other = nullptr, const int nwords = 0,
+                                               const bool skip0 = false) {
   typedef Mem<G> M;
+  const bool Z0 = CZ && skip0;  // the lowest rank is not emitted
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, T = blockDim.x;
   int hw = (cap - ((keep + 1) & ~1)) >> 1;         // counter words available above the kept slots
   typename M::ptr hist = M::add(buf, 2 * cap - 4 * hw);
@@ -380,7 +384,8 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
     __syncthreads();
     if (mini[17] == 0u) {
       const uint32_t Z = mini[18];  // rows with the lowest rank lead the sequence
-      for (uint32_t q = tid; q < Z; q += T) M::st16(M::add(buf, (int32_t)(q << 1)), 0u);
+      if (!Z0)
+        for (uint32_t q = tid; q < Z; q += T) M::st16(M::add(buf, (int32_t)(q << 1)), 0u);
       const int wpt = (bw + T - 1) / T, w0 = tid * wpt, w1 = min(w0 + wpt, bw);
       uint32_t mine = 0;
       for (int w = w0; w < w1; ++w) mine += __popc(M::ld32(M::add(bits, w << 2)));
@@ -393,7 +398,7 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
       if (lane == 31) descT[warp] = incl;
       __syncthreads();
       const uint32_t v = (lane < nwarps) ? descT[lane] : 0u;
-      uint32_t pos = Z + __reduce_add_sync(FULL, (lane < warp) ? v : 0u) + incl - mine;
+      uint32_t pos = (Z0 ? 0u : Z) + __reduce_add_sync(FULL, (lane < warp) ? v : 0u) + incl - mine;
       for (int w = w0; w < w1; ++w) {
         uint32_t m = M::ld32(M::add(bits, w << 2));
         while (m) {
@@ -450,7 +455,8 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
     if (EMIT) {
       uint32_t mine = 0;
       for (int w = w0; w < w1; ++w) {
-        const uint32_t c = M::ld32(M::add(hist, w << 2));
+        uint32_t c = M::ld32(M::add(hist, w << 2));
+        if (Z0 && k0 == 0 && w == 0) c &= 0xffff0000u;
         mine += (c & 0xffffu) + (c >> 16);
       }
       uint32_t incl = mine;
@@ -486,6 +492,10 @@ __device__ __forceinline__ uint32_t group_hist(typename Mem<G>::ptr buf, const i
           }
         }
         if (EMIT) {
+          if (Z0 && r == 0u) {
+            ties += (c * (c - (c ? 1u : 0u))) >> 1;
+            continue;
+          }
           if (c == 1u) {
             M::st16(M::add(buf, (int32_t)(pos << 1)), r);
           } else if (c > 1u) {
@@ -1103,12 +1113,111 @@ __device__ __forceinline__ void block_sum4(unsigned long long* red, int nwarps, 
   }
 }
 
+// The gather of the tier-0 short-vector kernel with y's lowest-rank keys left out (CZ, see DESIGN.md
+// section 2): seq'[q] for the x-present rows, i.e. rank_y[perm_x[q]] for q in [f, n) without the zero
+// keys, written behind the nonzero keys of x's first group.  A zero key is never the larger element of an
+// inversion, so leaving it out loses exactly the nonzero keys before it: the running write position when
+// it is met.  That sum goes to `zt` (this thread's share); returns len', the length of seq' (f < n: x has a
+// second group).  A round gives every warp 32 CH consecutive 8-key chunks, lane l takes chunks l, l + 32,
+// ... of them (coalesced loads; neighbouring lanes write about 8 slots apart, so the 16-bit stores of a
+// warp meet at most ~4 to a bank -- with CH consecutive chunks per lane they were 32 CH slots apart, 16 to a
+// bank).  The keys stay in registers across the round's one block scan; the chunks' nonzero counts go
+// through one warp scan as 16-bit pairs; the two block-scan arrays alternate between rounds.
+template <int CH>
+__device__ __forceinline__ uint32_t compact_gather(const uint32_t buf, const uint32_t rank_tbl,
+                                                   const uint16_t* __restrict__ permX, const int n, const int f,
+                                                   const uint32_t* mini18, uint32_t* descT, uint32_t* descB,
+                                                   const int nwarps, uint32_t& zt) {
+  static_assert(CH % 2 == 0, "chunk counts are scanned in pairs");
+  typedef Mem<false> M;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, T = blockDim.x;
+  auto rk = [&](uint32_t row) -> uint32_t { return M::ld16(M::add(rank_tbl, (int32_t)(row << 1))); };
+  const uint4* px8 = reinterpret_cast<const uint4*>(permX);
+  const int c_end = (n + 7) >> 3;
+  uint32_t base = 0xffffffffu;  // slots of seq' filled by the first group and earlier rounds
+  bool odd = false;
+  for (int c0 = f >> 3; c0 < c_end; c0 += CH * T, odd = !odd) {
+    const int cw = c0 + warp * 32 * CH + lane;  // this lane's chunk i is cw + 32 i
+    uint32_t k[CH][4];  // two keys per word; 0xffff: not a gathered position
+    uint32_t cnt[CH / 2] = {};  // nonzero keys of chunks 2m | 2m+1 (16 bits each)
+#pragma unroll
+    for (int i = 0; i < CH; ++i) {
+      const int c = cw + 32 * i, q0 = c << 3;
+      if (q0 >= f && q0 + 8 <= n) {
+        const uint4 pv = __ldg(px8 + c);
+        const uint32_t pw[4] = {pv.x, pv.y, pv.z, pv.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) k[i][j] = rk(pw[j] & 0xffffu) | (rk(pw[j] >> 16) << 16);
+      } else {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int qa = q0 + 2 * j, qb = qa + 1;
+          const uint32_t lo = (qa >= f && qa < n) ? rk(permX[qa]) : 0xffffu;
+          const uint32_t hi = (qb >= f && qb < n) ? rk(permX[qb]) : 0xffffu;
+          k[i][j] = lo | (hi << 16);
+        }
+      }
+      uint32_t nz = 0;
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        nz += (uint32_t)(((k[i][j] & 0xffffu) - 1u) < 0xfffeu) + (uint32_t)(((k[i][j] >> 16) - 1u) < 0xfffeu);
+      cnt[i >> 1] += (i & 1) ? nz << 16 : nz;
+    }
+    uint32_t incl[CH / 2];
+#pragma unroll
+    for (int m = 0; m < CH / 2; ++m) incl[m] = cnt[m];
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+#pragma unroll
+      for (int m = 0; m < CH / 2; ++m) {
+        const uint32_t t = __shfl_up_sync(FULL, incl[m], d);
+        if (lane >= d) incl[m] += t;
+      }
+    }
+    // slot of chunk i inside the warp's part: all lanes' earlier chunks + this chunk's earlier lanes
+    uint32_t off[CH], wtot = 0;
+#pragma unroll
+    for (int m = 0; m < CH / 2; ++m) {
+      const uint32_t tot = __shfl_sync(FULL, incl[m], 31), ex = incl[m] - cnt[m];
+      off[2 * m] = wtot + (ex & 0xffffu);
+      wtot += tot & 0xffffu;
+      off[2 * m + 1] = wtot + (ex >> 16);
+      wtot += tot >> 16;
+    }
+    uint32_t* desc = odd ? descB : descT;
+    if (lane == 31) desc[warp] = wtot;
+    __syncthreads();
+    if (base == 0xffffffffu) base = (uint32_t)f - *mini18;  // x's first group: f keys, mini[18] of them zero
+    const uint32_t v = (lane < nwarps) ? desc[lane] : 0u;
+    const uint32_t wbase = base + __reduce_add_sync(FULL, (lane < warp) ? v : 0u);
+    base += __reduce_add_sync(FULL, v);
+#pragma unroll
+    for (int i = 0; i < CH; ++i) {
+      uint32_t pos = wbase + off[i];
+#pragma unroll
+      for (int h = 0; h < 8; ++h) {
+        const uint32_t key = (k[i][h >> 1] >> ((h & 1) * 16)) & 0xffffu;
+        if (key - 1u < 0xfffeu) {
+          M::st16(M::add(buf, (int32_t)(pos << 1)), key);
+          ++pos;
+        } else if (key == 0u) {
+          zt += pos;
+        }
+      }
+    }
+  }
+  return base;
+}
+
 // PW: complete-observations mode (kt_fast use = "pairwise.complete.obs"): besides the global
 // counts the kernel takes the rows missing in either column out of the pair, see PairComplete.
 // IP: 0, or the compile-time run count KK of the in-place variant for long vectors (one sequence
 // buffer, keys in registers across a level, y's rank table read from global memory).
-template <int MAXT, int MINB, bool G, bool PW, int IP = 0>
+// CZ: tier 0 only -- pass A runs on the sequence without y's lowest-rank keys (compact_gather) for the pairs
+// where that takes a whole warp out of its levels.
+template <int MAXT, int MINB, bool G, bool PW, int IP = 0, bool CZ = false>
 __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledParams p) {
+  static_assert(!CZ || (!G && !PW && IP == 0), "the compacted sequence is for the shared-memory two-buffer kernel");
   typedef Mem<G> M;
   constexpr bool RG = G || IP != 0;    // rank table not staged
   constexpr int AQ = IP != 0 ? 2 : 4;  // bytes of the pass-A buffers in units of cap
@@ -1220,6 +1329,15 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
       const int m = XS.n_tied, nlg = XS.flags >> 8;
       const bool by_pass_b = nlg > 0 && p.tier == 2 && (long long)nlg * YS.n_groups > p.budget;
       uint32_t accB = 0;
+      // CZ: leave y's rank-0 keys out of pass A only where that takes a whole warp out of its levels (the
+      // compacting gather costs more than it saves otherwise).  Compacted, the first ceil(len' / R) ranges are
+      // swept, len' = n - (y's rank-0 rows); otherwise all but the floor(lead / R) leading ranges, where the
+      // leading block of zero keys is at most the smaller of the two columns' first groups.
+      bool cz = false;
+      if constexpr (CZ) {
+        const int y0 = max(YS.first_run, 1), lead_max = min(XS.first_run, y0);
+        cz = ((n - y0 + kkc - 1) / kkc + 31) / 32 < nwarps - lead_max / kkc / 32;
+      }
       if constexpr (!RG) {
         if (m > 0 && !by_pass_b)  // keys: 2 m <= 2 cap bytes, the still empty sequence buffer
           small_groups_direct(bufA, m, p.trow + (size_t)xcol * p.nstride, p.tord + (size_t)xcol * p.nstride,
@@ -1232,18 +1350,25 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
                                                   sm.fmask, fmask_words(nwarps, kkc) / 3, sm.descT, sm.mini + 16,
                                                   nwarps, p.gstart + (size_t)ycol * p.gstride, YS.n_na, pwy);
         else
-          ties += group_hist<G, true, false, RG>(bufA, cap, f, f, YS.n_groups, permX, rank_tbl, rankY_g, sm.mini,
+          ties += group_hist<G, true, false, RG, CZ>(bufA, cap, f, f, YS.n_groups, permX, rank_tbl, rankY_g, sm.mini,
                                                    sm.fmask, fmask_words(nwarps, kkc) / 3, sm.descT, sm.mini + 16,
                                                    nwarps, nullptr, 0, pwy,
                                                    8 * YS.n_tied <= n,  // y (nearly) tie-free: one bit per rank
-                                                   fbXg, sm.nabY, nwords);
+                                                   fbXg, sm.nabY, nwords, cz);
       }
       if (PW && YS.n_na > 0)  // the missing rows of y over the ranks of x (read from global memory)
         group_hist<G, false, true, true>(bufA, cap, f, YS.n_na, XS.n_groups, p.perm + (size_t)ycol * p.nstride,
                                          rank_tbl, p.rank + (size_t)xcol * p.nstride, sm.mini, sm.fmask,
                                          fmask_words(nwarps, kkc) / 3, sm.descT, sm.mini + 16, nwarps,
                                          p.gstart + (size_t)xcol * p.gstride, XS.n_na, pwx);
-      if (STG) {
+      uint32_t len = (uint32_t)cap, zt = 0u;  // CZ: length of seq', this thread's share of the zero term
+      if constexpr (CZ) {
+        if (cz)
+          len = compact_gather<4>(bufA, rank_tbl, permX, n, f, sm.mini + 18, sm.descT,
+                                  reinterpret_cast<uint32_t*>(sm.descB), nwarps, zt);
+      }
+      if (CZ && cz) {
+      } else if (STG) {
         staged_gather(smem_addr(sm.region_ptr), stage_tbl, stage_rows, permX, rankY_g, n, p.nstride, cap, padA, mbar, tma_phase);
       } else {  // seq[q] = rank_y[perm_x[q]] for q >= f, eight positions per thread and step
         auto rk = [&](uint32_t row) -> uint32_t {
@@ -1293,14 +1418,15 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
                                       reinterpret_cast<uint32_t*>(sm.red), sm.fmask, fmask_words(nwarps, kkc) / 3,
                                       sm.descT, sm.mini + 16, nwarps);
       }
-      unsigned long long accA = 0;
-      const uint32_t lead = sm.mini[18];  // published by the barrier after the gather
+      unsigned long long accA = zt;
+      // published by the barrier after the gather; a compacted sequence (len' < n <= cap) has no zero keys
+      const uint32_t lead = (CZ && len < (uint32_t)cap) ? 0u : sm.mini[18];
       if (IP != 0)
         count_pass_inplace<(IP != 0 ? IP : 1)>(smem_addr(sm.region_ptr), nwarps, L, sm.descT,
                                                reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc, accA, lead);
       else
-        count_pass<G>(bufA, bufB16, kk, nwarps, L, sm.descT, reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc, accA,
-                      lead);
+        count_pass<G, CZ>(bufA, bufB16, kk, nwarps, L, sm.descT, reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc,
+                          accA, lead, len);
       if (IP == 0 && m > 0 && by_pass_b) {
         const int kkB = (((m + 31) >> 5) + nwarps - 1) / nwarps;
         const int capB = (nwarps * kkB) << 5;
@@ -1868,9 +1994,9 @@ TiledShape tiled_shape(int64_t n, int tier, int64_t wstride, int n_sm, int64_t n
 
 namespace {
 
-template <int MAXT, int MINB, bool G, bool PW = false, int IP = 0>
+template <int MAXT, int MINB, bool G, bool PW = false, int IP = 0, bool CZ = false>
 int tiled_occupancy(int threads, size_t smem) {
-  auto kern = pairs_tiled_kernel<MAXT, MINB, G, PW, IP>;
+  auto kern = pairs_tiled_kernel<MAXT, MINB, G, PW, IP, CZ>;
   if (threads > MAXT) return 0;
   // always the architectural maximum, never the shape's own need: the attribute is per device, and two
   // host threads driving plans of different shapes on one device must not shrink it under each other
@@ -1890,14 +2016,17 @@ int tiled_occupancy(int threads, size_t smem) {
   return per_sm;
 }
 
-template <int MAXT, int MINB, bool G, bool PW = false, int IP = 0>
+template <int MAXT, int MINB, bool G, bool PW = false, int IP = 0, bool CZ = false>
 int launch_tiled_variant(const TiledParams& p, int threads, long long grid, size_t smem, cudaStream_t stream) {
-  pairs_tiled_kernel<MAXT, MINB, G, PW, IP><<<(unsigned)grid, threads, smem, stream>>>(p);
+  pairs_tiled_kernel<MAXT, MINB, G, PW, IP, CZ><<<(unsigned)grid, threads, smem, stream>>>(p);
   return launch_status(1);
 }
 
 // Three register classes of the same code (64 / 40 / 32 registers per thread): take the roomiest
 // one unless a tighter class keeps clearly more threads resident for this shared-memory footprint.
+template <bool G, bool CZ>
+int launch_tiled_cls(const TiledParams& p, const TiledShape& sh, size_t smem, int n_sm, cudaStream_t stream);
+
 template <bool G>
 int launch_tiled_g(TiledParams& p, const TiledShape& sh, size_t smem, int n_sm, cudaStream_t stream) {
   const int threads = 32 * sh.warps;
@@ -1916,9 +2045,19 @@ int launch_tiled_g(TiledParams& p, const TiledShape& sh, size_t smem, int n_sm, 
     if (grid < 1) grid = 1;
     return launch_tiled_variant<1024, 1, G, true>(p, threads, grid, smem, stream);
   }
-  const int o64 = tiled_occupancy<1024, 1, G>(threads, smem);
-  const int o40 = tiled_occupancy<512, 3, G>(threads, smem);
-  const int o32 = tiled_occupancy<1024, 2, G>(threads, smem);
+  // tier 0 in shared memory with 8 or more warps may run pass A on the sequence without y's lowest-rank keys
+  // (decided per pair).  Below that the compacting instantiation measured slower on a B200 although it compacts
+  // nothing there (1-4 warps at n = 2 000 ... 6 887: 0.4-1.7 %); at 16 warps (n = 20 000) it gains 4.7 %.
+  if (!G && p.tier == 0 && sh.warps >= 8) return launch_tiled_cls<G, !G>(p, sh, smem, n_sm, stream);
+  return launch_tiled_cls<G, false>(p, sh, smem, n_sm, stream);
+}
+
+template <bool G, bool CZ>
+int launch_tiled_cls(const TiledParams& p, const TiledShape& sh, size_t smem, int n_sm, cudaStream_t stream) {
+  const int threads = 32 * sh.warps;
+  const int o64 = tiled_occupancy<1024, 1, G, false, 0, CZ>(threads, smem);
+  const int o40 = tiled_occupancy<512, 3, G, false, 0, CZ>(threads, smem);
+  const int o32 = tiled_occupancy<1024, 2, G, false, 0, CZ>(threads, smem);
   // the tighter classes spill: they have to buy at least a quarter more resident CTAs
   int cls = 0, best = o64;
   if (4 * o40 >= 5 * best) { cls = 1; best = o40; }
@@ -1937,9 +2076,9 @@ int launch_tiled_g(TiledParams& p, const TiledShape& sh, size_t smem, int n_sm, 
   if (grid > p.n_units) grid = p.n_units;
   if (G && grid > sh.scratch_ctas) grid = sh.scratch_ctas;
   if (grid < 1) grid = 1;
-  if (cls == 2) return launch_tiled_variant<1024, 2, G>(p, threads, grid, smem, stream);
-  if (cls == 1) return launch_tiled_variant<512, 3, G>(p, threads, grid, smem, stream);
-  return launch_tiled_variant<1024, 1, G>(p, threads, grid, smem, stream);
+  if (cls == 2) return launch_tiled_variant<1024, 2, G, false, 0, CZ>(p, threads, grid, smem, stream);
+  if (cls == 1) return launch_tiled_variant<512, 3, G, false, 0, CZ>(p, threads, grid, smem, stream);
+  return launch_tiled_variant<1024, 1, G, false, 0, CZ>(p, threads, grid, smem, stream);
 }
 
 }  // namespace
