@@ -1018,7 +1018,9 @@ int launch_columns(const double* d_data, int64_t ld, const double* d_global_na, 
   int launches = 0;
   // tie-group thresholds (icikt_common.cuh); the environment overrides are for tuning sweeps
   int large_tie = kLargeTie, direct_budget = kDirectBudget;
-  if (const char* e = getenv("ICIKT_LARGE_TIE")) large_tie = std::min(2048, std::max(2, atoi(e)));
+  // at least ceil(n / 512): a column then has fewer large groups than the lgrp table's 512 slots
+  if (const char* e = getenv("ICIKT_LARGE_TIE"))
+    large_tie = std::min(2048, std::max(std::max(2, (n + kLargeStride / 2 - 1) / (kLargeStride / 2)), atoi(e)));
   if (const char* e = getenv("ICIKT_DIRECT_BUDGET")) direct_budget = std::min(63, std::max(0, atoi(e)));
   // the bit arrays are written in full (words below n32/32) by the kernels below; the padding
   // words up to wstride were zeroed once when the plan was created

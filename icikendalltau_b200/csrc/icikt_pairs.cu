@@ -590,7 +590,9 @@ __device__ __forceinline__ void small_groups_direct(const uint32_t keys, const i
 // after the gather.  The rows of a tie group are consecutive in x order, so the keys of the rows behind a
 // row are the ones behind its position (K1's `tend` table: position in sorted order of every list entry);
 // no second lookup of the ranks through L2, no copy of the keys.  Large groups and the first group occupy
-// other positions, so nothing this routine reads is rewritten before pass A's first barrier.
+// other positions.  Ends with a barrier: for L <= 4 pass A starts with its low-nibble level, whose warps
+// park their totals over the first keys of their ranges before any barrier, while slower warps would still
+// read those keys here.
 template <bool G>
 __device__ __forceinline__ void small_groups_inplace(typename Mem<G>::ptr seq, const int m,
                                                      const uint32_t* __restrict__ tord,
@@ -615,6 +617,7 @@ __device__ __forceinline__ void small_groups_inplace(typename Mem<G>::ptr seq, c
     inv += (uint32_t)walk - ge;        // other < mine
     ties += ge + le - (uint32_t)walk;  // other == mine
   }
+  __syncthreads();
 }
 
 // Large tie groups of x (other than the first): their rows' y-ranks, already gathered into the

@@ -80,10 +80,15 @@ def test_nearly_all_missing():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("n", [3000, 20000])
-def test_lengths_around_range_multiples(n):
+def test_lengths_around_range_multiples(n, monkeypatch):
     """y's present rows (pass A's length without the zero keys) just below, on and just above multiples of
-    the thread range R of the launch shape and of 8"""
-    R = 8 * _lib.launch_shape(n, 0)["runs"]
+    the thread range R of the launch shape and of 8.  The shape is the one of a large job, pinned with
+    ICIKT_WARPS: these few pairs would otherwise plan a wider one with another R."""
+    shape = _lib.launch_shape(n, 0)
+    monkeypatch.setenv("ICIKT_WARPS", str(shape["warps"]))
+    _lib.release_workspace()
+    assert _lib.launch_shape(n, 0) == shape
+    R = 8 * shape["runs"]
     lens = set()
     for m in (R, 8, 32 * R):
         for k in (1, 2, 7, n // m - 1):
@@ -96,6 +101,7 @@ def test_lengths_around_range_multiples(n):
         part = lens[i:i + 4]
         miss = [n - v for v in part] + [n // 4]
         check(censored(n, len(miss), miss, seed=100 + i), with_oracle=(n <= 3000))
+    _lib.release_workspace()
 
 
 @pytest.mark.gpu
