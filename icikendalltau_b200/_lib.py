@@ -39,6 +39,8 @@ EXPORTS = [
     "icikt_matrices_multi_csc", "icikt_pairwise_completeness_csc",
     "icikt_all_pairs_edges", "icikt_all_pairs_edges_csc", "icikt_edges_count", "icikt_edges_copy",
     "icikt_edges_free", "icikt_all_pairs_topk", "icikt_all_pairs_topk_csc",
+    "icikt_all_pairs_edges_multi", "icikt_all_pairs_edges_multi_csc", "icikt_all_pairs_topk_multi",
+    "icikt_all_pairs_topk_multi_csc",
 ]
 NSTATUS = 10
 
@@ -178,6 +180,13 @@ def load():
     L.icikt_all_pairs_topk.restype = ctypes.c_int
     L.icikt_all_pairs_topk_csc.argtypes = csc + L.icikt_all_pairs_topk.argtypes[4:]
     L.icikt_all_pairs_topk_csc.restype = ctypes.c_int
+    # the multi-device twins of the filtered calls: (devices, n_devices) after opts
+    for name in ("icikt_all_pairs_edges", "icikt_all_pairs_topk"):
+        a = getattr(L, name).argtypes
+        for sfx, lead in (("_multi", a[:7]), ("_multi_csc", csc + a[4:7])):
+            f = getattr(L, name + sfx)
+            f.argtypes = lead + [_ip, ctypes.c_int32] + a[7:]
+            f.restype = ctypes.c_int
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -349,25 +358,38 @@ def _bound(v):
     return float("nan") if v is None else float(v)
 
 
-def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, **opt_kw):
+def _devices_args(devices):
+    """(suffix of the entry point, its (devices, n_devices) arguments, the array that owns them): the single-device
+    call for devices None, otherwise its _multi twin"""
+    if devices is None:
+        return "", (), None
+    dev = np.ascontiguousarray(list(devices), dtype=np.int32)
+    return "_multi", (_ptr(dev, _ip), int(dev.size)), dev
+
+
+def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, devices=None,
+              **opt_kw):
     """icikt_all_pairs_edges: all pairs, filtered on the device, as a long table of the pairs that pass.
 
     A pair is kept iff it is not degenerate, abs(cor) >= min_abs_cor and pvalue <= max_pvalue (a bound of None is
     no condition), with cor = raw / max(taumax over all pairs) if scale_max else raw.  Rows are in the pair order
     of run_pairs, and every field is bit for bit run_pairs' for that pair.  data may be a scipy.sparse matrix
     (-> icikt_all_pairs_edges_csc).  max_edges > 0 raises IciktError(ERR_LIMIT) when more pairs pass.
+    devices: list of CUDA ordinals -> icikt_all_pairs_edges_multi(_csc): every device walks a contiguous slice of the
+    pair order; the result is bit for bit the single-device one.
     Returns a dict of NumPy arrays i, j (int32), cor, raw, pvalue, taumax, completeness, plus max_taumax and
     timings."""
     L = load()
     lead, sfx, n, C, keep_alive = _matrix_args(data)
+    msfx, dargs, dev = _devices_args(devices)
     o = make_opts(**opt_kw)
     f = EdgeFilter(_bound(min_abs_cor), _bound(max_pvalue), int(bool(scale_max)), 0, int(max_edges))
     h = ctypes.c_void_p()
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(getattr(L, "icikt_all_pairs_edges" + sfx)(*lead, gp, ng, ctypes.byref(o), ctypes.byref(f), ctypes.byref(h),
-                                                    ctypes.byref(mx), ctypes.byref(t)))
+    check(getattr(L, "icikt_all_pairs_edges" + msfx + sfx)(*lead, gp, ng, ctypes.byref(o), *dargs, ctypes.byref(f),
+                                                           ctypes.byref(h), ctypes.byref(mx), ctypes.byref(t)))
     try:
         m = int(L.icikt_edges_count(h))
         out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
@@ -379,19 +401,22 @@ def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=T
     return out
 
 
-def run_topk(data, global_na=(), k=10, by="abs", scale_max=True, **opt_kw):
+def run_topk(data, global_na=(), k=10, by="abs", scale_max=True, devices=None, **opt_kw):
     """icikt_all_pairs_topk: every column's k best partners over all pairs, selected on the device.
 
     The candidates of column c are the columns d != c whose pair is not degenerate, ranked by abs(raw) (by="abs")
     or raw (by="signed") descending, then d ascending; column c keeps its first min(k, #candidates), best first.
     Every field is bit for bit run_pairs' for that pair, cor = raw / max_taumax if scale_max else raw.  data may be
-    a scipy.sparse matrix (-> icikt_all_pairs_topk_csc).  Returns a dict with index (C, k) int32 (-1 where
+    a scipy.sparse matrix (-> icikt_all_pairs_topk_csc).  devices: list of CUDA ordinals ->
+    icikt_all_pairs_topk_multi(_csc): every device walks a contiguous slice of the pair order and the devices merge
+    their lists, bit for bit the single-device result.  Returns a dict with index (C, k) int32 (-1 where
     unused), cor, raw, pvalue, taumax, completeness (C, k) float64 (NaN where unused), n_neighbors (C,) int32,
     max_taumax and timings."""
     if by not in TOPK_BY:
         raise ValueError(f"by must be one of {sorted(TOPK_BY)}")
     L = load()
     lead, sfx, n, C, keep_alive = _matrix_args(data)
+    msfx, dargs, dev = _devices_args(devices)
     o = make_opts(**opt_kw)
     k = int(k)
     kk = k if 1 <= k <= TOPK_MAX else 0  # a k the library refuses gets no arrays
@@ -402,10 +427,11 @@ def run_topk(data, global_na=(), k=10, by="abs", scale_max=True, **opt_kw):
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(getattr(L, "icikt_all_pairs_topk" + sfx)(*lead, gp, ng, ctypes.byref(o), k, TOPK_BY[by],
-                                                   int(bool(scale_max)), _ptr(out["index"]), _ptr(out["n_neighbors"]),
-                                                   *(_ptr(out[name]) for name in EDGE_NAMES), ctypes.byref(mx),
-                                                   ctypes.byref(t)))
+    check(getattr(L, "icikt_all_pairs_topk" + msfx + sfx)(*lead, gp, ng, ctypes.byref(o), *dargs, k, TOPK_BY[by],
+                                                          int(bool(scale_max)), _ptr(out["index"]),
+                                                          _ptr(out["n_neighbors"]),
+                                                          *(_ptr(out[name]) for name in EDGE_NAMES), ctypes.byref(mx),
+                                                          ctypes.byref(t)))
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 

@@ -251,7 +251,8 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     diag_good are subject to the same mask).  Over all pairs the selection runs on the device window by window
     (_lib.run_edges), so neither the result nor the device memory grows with the number of pairs; degenerate
     pairs never pass and raise no warning there.  max_edges: raise IciktError (ERR_LIMIT) when more computed
-    pairs than that pass.
+    pairs than that pass.  The filtered table over several GPUs is _lib.run_edges(..., devices=[...]), which
+    returns the same rows as one GPU.
     """
     filtered = min_abs_cor is not None or max_pvalue is not None
     if filtered and return_matrix:
@@ -365,13 +366,14 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
 
 
 def ici_kendalltau_topk(data_matrix, k, by="abs", global_na=(np.nan, np.inf, 0), perspective="global",
-                        scale_max=True, alternative="two.sided", continuity=False, colnames=None, device=0):
+                        scale_max=True, alternative="two.sided", continuity=False, colnames=None, device=0, n_gpus=1):
     """Every sample's k most correlated partners (a kNN table), over all pairs of a features x samples matrix.
 
     The candidates of sample c are the samples d != c whose pair is not degenerate, ranked by abs(raw) (by="abs")
     or raw (by="signed") descending, then by column position; c keeps its first min(k, #candidates), best first.
-    The selection runs on one GPU window by window (_lib.run_topk), so neither the result nor the device memory
-    grows with the number of pairs; degenerate pairs raise no warning.  Values are those of ici_kendalltau for the
+    The selection runs window by window (_lib.run_topk), so neither the result nor the device memory grows with the
+    number of pairs; degenerate pairs raise no warning.  n_gpus > 1 spreads the pair order over GPUs 0..n_gpus-1 of
+    the box in one library call (`device` is then not used); the lists are the same as on one GPU.  Values are those of ici_kendalltau for the
     same pair, cor = raw / max(taumax over all pairs) if scale_max else raw.
 
     Returns a dict of (C, k) arrays `index` (int32, -1 where unused), `neighbors` (column names, None where
@@ -386,8 +388,10 @@ def ici_kendalltau_topk(data_matrix, k, by="abs", global_na=(np.nan, np.inf, 0),
     global_na = [float(v) for v in global_na]
     log.info("Running correlations ...")
     t1 = time.perf_counter()
-    r = _lib.run_topk(data, global_na, int(k), by, scale_max, perspective=perspective, alternative=alternative,
-                      continuity=continuity, device=device)
+    kw = dict(perspective=perspective, alternative=alternative, continuity=continuity, device=device)
+    if n_gpus > 1:
+        kw["devices"] = range(n_gpus)
+    r = _lib.run_topk(data, global_na, int(k), by, scale_max, **kw)
     run_time = time.perf_counter() - t1
     nm = np.empty(len(names) + 1, dtype=object)  # the last entry, None, is what index -1 picks
     for c, v in enumerate(names):

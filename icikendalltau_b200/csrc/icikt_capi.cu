@@ -5,10 +5,12 @@
 // column chunks upload behind the pair launches of earlier chunks, finished row blocks of the
 // results leave behind later ones.
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <string>
@@ -264,6 +266,11 @@ struct icikt_plan {
   int32_t* d_tidx = nullptr;   // [C k]
   double* d_tlist = nullptr;   // 4 x [C k]: raw, pvalue, taumax, completeness
   int topk_cap = 0;
+  // Top-k over several devices (icikt_all_pairs_topk_multi): this device's block of columns of the merged lists
+  int32_t* d_mn = nullptr;     // [C] entries kept per column of the block
+  int32_t* d_midx = nullptr;   // [merge_cap]
+  double* d_mlist = nullptr;   // 4 x [merge_cap]: raw, pvalue, taumax, completeness
+  size_t merge_cap = 0;
 
   cudaEvent_t ev[9]{};
   icikt_timings tm{};
@@ -333,6 +340,9 @@ void free_plan(icikt_plan* p) {
   cudaFree(p->d_tcol);
   cudaFree(p->d_tidx);
   cudaFree(p->d_tlist);
+  cudaFree(p->d_mn);
+  cudaFree(p->d_midx);
+  cudaFree(p->d_mlist);
   for (auto& e : p->ev)
     if (e) cudaEventDestroy(e);
   for (auto& e : p->sync_ev)
@@ -1434,6 +1444,7 @@ static bool want_staged(int64_t n, int64_t C, const icikt_opts& o, bool all_pair
 static icikt_plan* g_cached = nullptr;
 static icikt_plan* g_cached_multi[64] = {};  // one slot per worker of icikt_all_pairs_multi
 static icikt_plan* g_cached_edges = nullptr;    // the filtered call's (its pair buffers hold one window)
+static icikt_plan* g_cached_wmulti[kMaxMatrixDevices] = {};  // one slot per worker of the filtered calls' multi twins
 static std::mutex g_cache_mu;
 
 static bool cache_matches(const icikt_plan* p, int64_t n, int64_t C, const icikt_opts& o, bool staged) {
@@ -1526,6 +1537,8 @@ void icikt_release_workspace(void) {
   if (g_cached) { icikt_plan_destroy(g_cached); g_cached = nullptr; }
   if (g_cached_edges) { icikt_plan_destroy(g_cached_edges); g_cached_edges = nullptr; }
   for (icikt_plan*& s : g_cached_multi)
+    if (s) { icikt_plan_destroy(s); s = nullptr; }
+  for (icikt_plan*& s : g_cached_wmulti)
     if (s) { icikt_plan_destroy(s); s = nullptr; }
 }
 
@@ -1756,6 +1769,22 @@ static int ensure_topk_buffers(icikt_plan* p, int64_t W, int k) {
   return ICIKT_OK;
 }
 
+// the merged lists of a block of columns (top-k over several devices): `entries` = columns of the block x k
+static int ensure_merge_buffers(icikt_plan* p, size_t entries) {
+  if (!p->d_mn) ECK(dmalloc(&p->d_mn, (size_t)p->C));
+  if (entries > p->merge_cap) {
+    cudaFree(p->d_midx);
+    cudaFree(p->d_mlist);
+    p->d_midx = nullptr;
+    p->d_mlist = nullptr;
+    p->merge_cap = 0;
+    ECK(dmalloc(&p->d_midx, entries));
+    ECK(dmalloc(&p->d_mlist, 4 * entries));
+    p->merge_cap = entries;
+  }
+  return ensure_stage(p);
+}
+
 // room for `need` units in both window unit buffers (device and pinned host)
 static int ensure_window_units(icikt_plan* p, size_t need) {
   if (need <= p->wunit_cap) return ICIKT_OK;
@@ -1783,25 +1812,30 @@ struct WalkTotals {
   unsigned long long bits = 0;
 };
 
-// The window walk of the filtered calls, on a plan whose pair buffers hold W pairs: upload and K1 once, then the
-// pair order in windows of W.  Window w is enqueued (units, K2, K3, `select`, the readback of the maximum so
-// far) before the host waits for window w - 1 and runs `collect` for it; d_maxbits is not reset between
-// windows, so K3's atomicMax leaves that maximum.  select(w, b, units, n_units, n_slots) enqueues the
-// selection of window w on p->stream (b: its buffer, 0 or 1); collect(w, b) runs once that has completed.
+// upload and K1 of the single-device filtered calls, ahead of their window walk
+static int window_columns(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na) {
+  const int rc = upload_columns(p, s, 0, p->C);
+  return rc == ICIKT_OK ? plan_columns_impl(p, global_na, n_global_na, 0, p->C, true) : rc;
+}
+
+// The window walk of the filtered calls, on a plan whose pair buffers hold W pairs and whose columns are prepared
+// (K1 enqueued): pairs [first, last) of the pair order in windows of W.  Window w is enqueued (units, K2, K3,
+// `select`, the readback of the maximum so far) before the host waits for window w - 1 and runs `collect` for it;
+// d_maxbits is not reset between windows, so K3's atomicMax leaves that maximum.  select(w, b, units, n_units,
+// n_slots) enqueues the selection of window w on p->stream (b: its buffer, 0 or 1); collect(w, b) runs once that
+// has completed.
 template <class Select, class Collect>
-static int walk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
-                        int64_t ptot, int64_t W, WalkTotals& tot, Select&& select, Collect&& collect) {
-  int rc = upload_columns(p, s, 0, p->C);
-  if (rc == ICIKT_OK) rc = plan_columns_impl(p, global_na, n_global_na, 0, p->C, true);
-  if (rc != ICIKT_OK) return rc;
+static int walk_windows(icikt_plan* p, int64_t first, int64_t last, int64_t W, WalkTotals& tot, Select&& select,
+                        Collect&& collect) {
   tot.launches = p->tm.n_launches;
   CK(cudaMemsetAsync(p->d_maxbits, 0, sizeof(unsigned long long), p->stream));
-  const int64_t nwin = (ptot + W - 1) / W, ptri = tri_pairs(p->C), slots = (int64_t)p->n_sm * 2;
+  const int64_t nwin = (last - first + W - 1) / W, ptri = tri_pairs(p->C), slots = (int64_t)p->n_sm * 2;
   std::vector<PairUnit> U;
+  int rc = ICIKT_OK;
 
   auto enqueue = [&](int64_t w) -> int {
     const int b = (int)(w & 1);
-    const int64_t lo = w * W, hi = std::min(ptot, lo + W);
+    const int64_t lo = first + w * W, hi = std::min(last, lo + W);
     int32_t row = 0, col = 0;
     if (lo < ptri) icikt_pair_from_index(p->C, 0, lo, &row, &col);
     U.clear();
@@ -1863,21 +1897,29 @@ static int finish_walk(icikt_plan* p, const WalkTotals& tot, float d2h_ms, icikt
   return ICIKT_OK;
 }
 
-// The filtered call: per window, the edge selection and the readback of its row count; once the host has waited
-// for a window, its rows are copied out on the copy stream and the rows held are re-trimmed against the new
-// maximum.
-static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
-                        const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
-                        icikt_timings* timings) {
-  int rc = ensure_edge_buffers(p, W);
-  if (rc != ICIKT_OK) return rc;
+// The rows all walkers of one filtered call hold, for max_edges: one walker on one device, one per device in the
+// multi-device call.  A walker that takes the sum over the limit raises `stop`, and the others fail at their next
+// window boundary.
+struct EdgeHeld {
+  std::atomic<int64_t> total{0};
+  std::atomic<bool> stop{false};
+};
+
+static int edge_limit_fail(const icikt_edge_filter& f, int64_t held, const std::string& where) {
+  return fail(ICIKT_ERR_LIMIT, "more than max_edges = " + std::to_string(f.max_edges) + " pairs pass the filter (" +
+                                   std::to_string(held) + where + ")");
+}
+
+// The filtered call's walk over pairs [first, last): per window, the edge selection and the readback of its row
+// count; once the host has waited for a window, its rows are copied out on the copy stream and appended to `rows`,
+// and the rows held are re-trimmed against the new maximum (this walk's own: at most the final one, so the rows
+// stay a superset of the final edges).  The plan's edge buffers hold windows of W pairs.
+static int edge_walk(icikt_plan* p, const icikt_edge_filter& f, int64_t first, int64_t last, int64_t W,
+                     std::vector<EdgeRow>& rows, EdgeHeld& held, WalkTotals& tot, float& d2h_ms) {
   const double t = f.min_abs_cor;
   const bool scale = f.scale_max != 0;
   const bool retrim = scale && t == t;
-  const int64_t nwin = (ptot + W - 1) / W;
-  std::vector<EdgeRow>& rows = res->rows;
-  WalkTotals tot;
-  float d2h_ms = 0.f;
+  const int64_t nwin = (last - first + W - 1) / W;
   unsigned long long trimmed_bits = 0;
 
   auto select = [&](int64_t, int b, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
@@ -1906,8 +1948,10 @@ static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* glob
   };
 
   auto collect = [&](int64_t w, int b) -> int {
+    if (held.stop) return edge_limit_fail(f, held.total, " held when another device reached the limit");
     const unsigned long long cnt = p->h_estat[2 * b];
     const unsigned long long bits = tot.bits;
+    const size_t before = rows.size();
     if (cnt) {
       const size_t old = rows.size();
       try {
@@ -1928,26 +1972,51 @@ static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* glob
                  rows.end());
       trimmed_bits = bits;
     }
-    if (f.max_edges > 0 && (int64_t)rows.size() > f.max_edges)
-      return fail(ICIKT_ERR_LIMIT, "more than max_edges = " + std::to_string(f.max_edges) + " pairs pass the filter (" +
-                                       std::to_string(rows.size()) + " held after " + std::to_string(w + 1) + " of " +
-                                       std::to_string(nwin) + " windows)");
+    const int64_t sum = held.total += (int64_t)rows.size() - (int64_t)before;
+    if (f.max_edges > 0 && sum > f.max_edges) {
+      held.stop = true;
+      return edge_limit_fail(f, sum, " held after " + std::to_string(w + 1) + " of " + std::to_string(nwin) + " windows");
+    }
     return ICIKT_OK;
   };
 
-  rc = walk_windows(p, s, global_na, n_global_na, ptot, W, tot, select, collect);
-  if (rc != ICIKT_OK) return rc;
-  // the exact predicate with the final maximum
-  const double M = max_of_bits(tot.bits);
+  return walk_windows(p, first, last, W, tot, select, collect);
+}
+
+// The end of the filtered call, on one device or several: the rows held, in pair order, get the exact predicate with
+// the final maximum M, the max_edges check and cor.
+static int edge_result(icikt_edges* res, const icikt_edge_filter& f, double M) {
+  std::vector<EdgeRow>& rows = res->rows;
+  const double t = f.min_abs_cor;
+  const bool scale = f.scale_max != 0;
   if (scale && t == t)
     rows.erase(std::remove_if(rows.begin(), rows.end(), [&](const EdgeRow& r) { return !edge_keep_final(r.raw, t, true, M); }),
                rows.end());
-  if (f.max_edges > 0 && (int64_t)rows.size() > f.max_edges)
-    return fail(ICIKT_ERR_LIMIT, "more than max_edges = " + std::to_string(f.max_edges) + " pairs pass the filter (" +
-                                     std::to_string(rows.size()) + ")");
-  res->cor.resize(rows.size());
+  if (f.max_edges > 0 && (int64_t)rows.size() > f.max_edges) return edge_limit_fail(f, (int64_t)rows.size(), "");
+  try {
+    res->cor.resize(rows.size());
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for cor");
+  }
   for (size_t k = 0; k < rows.size(); ++k) res->cor[k] = scale ? rows[k].raw / M : rows[k].raw;
-  rc = finish_walk(p, tot, d2h_ms, timings);
+  return ICIKT_OK;
+}
+
+// The filtered call on one device: upload, K1, the walk over the whole pair order, the final trim.
+static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
+                        const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
+                        icikt_timings* timings) {
+  int rc = ensure_edge_buffers(p, W);
+  if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na);
+  if (rc != ICIKT_OK) return rc;
+  WalkTotals tot;
+  float d2h_ms = 0.f;
+  EdgeHeld held;
+  rc = edge_walk(p, f, 0, ptot, W, res->rows, held, tot, d2h_ms);
+  if (rc != ICIKT_OK) return rc;
+  const double M = max_of_bits(tot.bits);
+  rc = edge_result(res, f, M);
+  if (rc == ICIKT_OK) rc = finish_walk(p, tot, d2h_ms, timings);
   if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = M;
   return ICIKT_OK;
@@ -1962,17 +2031,11 @@ struct TopkOut {
   double *cor, *raw, *pvalue, *taumax, *completeness;
 };
 
-static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na, int k,
-                        int by, bool scale, int64_t ptot, int64_t W, const TopkOut& out, double* max_taumax,
-                        icikt_timings* timings) {
-  int rc = ensure_topk_buffers(p, W, k);
-  if (rc != ICIKT_OK) return rc;
+// The top-k call's walk over pairs [first, last): the lists start empty and every window's candidates are merged
+// into them on the device.  The plan's top-k buffers hold windows of W pairs and lists of k entries.
+static int topk_walk(icikt_plan* p, int k, int by, int64_t first, int64_t last, int64_t W, WalkTotals& tot) {
   const int64_t C = p->C, ck = C * k;
   CK(cudaMemsetAsync(p->d_tcol, 0, sizeof(TopkCol) * (size_t)C, p->stream));
-  double* d_raw = p->d_tlist;
-  double* d_field[3] = {p->d_tlist + ck, p->d_tlist + 2 * ck, p->d_tlist + 3 * ck};
-  WalkTotals tot;
-
   auto select = [&](int64_t, int b, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
     TopkSelect ts;
     ts.units = units;
@@ -1991,55 +2054,84 @@ static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* glob
     ts.cand = p->d_tcand;
     ts.col = p->d_tcol;
     ts.idx = p->d_tidx;
-    ts.raw = d_raw;
-    ts.pv = d_field[0];
-    ts.tm = d_field[1];
-    ts.comp = d_field[2];
+    ts.raw = p->d_tlist;
+    ts.pv = p->d_tlist + ck;
+    ts.tm = p->d_tlist + 2 * ck;
+    ts.comp = p->d_tlist + 3 * ck;
     const int l = launch_topk_select(ts, p->stream);
     if (l < 0) return launch_fail("top-k selection kernels");
     tot.launches += l;
     return ICIKT_OK;
   };
+  return walk_windows(p, first, last, W, tot, select, [](int64_t, int) { return ICIKT_OK; });
+}
 
-  rc = walk_windows(p, s, global_na, n_global_na, ptot, W, tot, select, [](int64_t, int) { return ICIKT_OK; });
-  if (rc != ICIKT_OK) return rc;
-  // the lists, once
-  std::vector<TopkCol> col;
-  std::vector<double> raw_own;
-  double* raw = out.raw;
+// raw for cor when the caller wants cor but not raw
+static int topk_raw_buffer(const TopkOut& out, int64_t ck, std::vector<double>& own, double** raw) {
+  *raw = out.raw;
+  if (out.raw || !out.cor) return ICIKT_OK;
   try {
-    col.resize((size_t)C);
-    if (!raw && out.cor) {
-      raw_own.resize((size_t)ck);
-      raw = raw_own.data();
-    }
+    own.resize((size_t)ck);
   } catch (const std::bad_alloc&) {
     return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
   }
-  CK(cudaEventRecord(p->ev[6], p->stream));
-  rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)C, p->stream);
-  if (rc == ICIKT_OK) rc = staged_copy_out(p, out.index, p->d_tidx, sizeof(int32_t) * (size_t)ck, p->stream);
-  if (rc == ICIKT_OK && raw) rc = staged_copy_out(p, raw, d_raw, sizeof(double) * (size_t)ck, p->stream);
-  double* host_field[3] = {out.pvalue, out.taumax, out.completeness};
-  for (int f = 0; f < 3 && rc == ICIKT_OK; ++f)
-    if (host_field[f]) rc = staged_copy_out(p, host_field[f], d_field[f], sizeof(double) * (size_t)ck, p->stream);
-  if (rc != ICIKT_OK) return rc;
-  CK(cudaEventRecord(p->ev[7], p->stream));
-  CK(cudaEventSynchronize(p->ev[7]));
-  const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
-  const double M = max_of_bits(tot.bits);
+  *raw = own.data();
+  return ICIKT_OK;
+}
+
+// The host's part of the top-k result once the lists of columns [0, C) are in the caller's arrays (raw: out.raw or
+// the buffer topk_raw_buffer gave): n_neighbors from held(c), cor = raw / M (scale) or raw, and the padding.
+template <class Held>
+static void topk_fill_host(const TopkOut& out, int64_t C, int k, Held&& held, const double* raw, bool scale, double M) {
   const double qnan = std::nan("");
   for (int64_t c = 0; c < C; ++c) {
-    const int64_t held = col[(size_t)c].n, base = c * k;
-    if (out.n_neighbors) out.n_neighbors[c] = (int32_t)held;
+    const int64_t h = held(c), base = c * k;
+    if (out.n_neighbors) out.n_neighbors[c] = (int32_t)h;
     if (out.cor)
-      for (int64_t r = 0; r < held; ++r) out.cor[base + r] = scale ? raw[base + r] / M : raw[base + r];
-    for (int64_t r = held; r < k; ++r) {
+      for (int64_t r = 0; r < h; ++r) out.cor[base + r] = scale ? raw[base + r] / M : raw[base + r];
+    for (int64_t r = h; r < k; ++r) {
       out.index[base + r] = -1;
       for (double* a : {out.cor, out.raw, out.pvalue, out.taumax, out.completeness})
         if (a) a[base + r] = qnan;
     }
   }
+}
+
+// The top-k call on one device: nothing comes back until the last window, then the lists are copied out once and
+// cor is formed with the final maximum.
+static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na, int k,
+                        int by, bool scale, int64_t ptot, int64_t W, const TopkOut& out, double* max_taumax,
+                        icikt_timings* timings) {
+  int rc = ensure_topk_buffers(p, W, k);
+  if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t C = p->C, ck = C * k;
+  WalkTotals tot;
+  rc = topk_walk(p, k, by, 0, ptot, W, tot);
+  if (rc != ICIKT_OK) return rc;
+  // the lists, once
+  std::vector<TopkCol> col;
+  std::vector<double> raw_own;
+  double* raw = nullptr;
+  try {
+    col.resize((size_t)C);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
+  }
+  rc = topk_raw_buffer(out, ck, raw_own, &raw);
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[6], p->stream));
+  rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)C, p->stream);
+  if (rc == ICIKT_OK) rc = staged_copy_out(p, out.index, p->d_tidx, sizeof(int32_t) * (size_t)ck, p->stream);
+  double* host_field[4] = {raw, out.pvalue, out.taumax, out.completeness};
+  for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
+    if (host_field[f]) rc = staged_copy_out(p, host_field[f], p->d_tlist + f * ck, sizeof(double) * (size_t)ck, p->stream);
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[7], p->stream));
+  CK(cudaEventSynchronize(p->ev[7]));
+  const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
+  const double M = max_of_bits(tot.bits);
+  topk_fill_host(out, C, k, [&](int64_t c) { return (int64_t)col[(size_t)c].n; }, raw, scale, M);
   rc = finish_walk(p, tot, d2h_ms, timings);
   if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = M;
@@ -2047,10 +2139,10 @@ static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* glob
 }
 #undef ECK
 
-// The plan of the filtered calls (cached in g_cached_edges; the caller holds g_cache_mu): pair buffers of one
-// window of W pairs.
-static int window_plan(int64_t n, int64_t C, int64_t W, const icikt_opts& o, icikt_plan** out) {
-  icikt_plan* p = g_cached_edges;
+// The plan of the filtered calls (cached in `slot`: g_cached_edges, or a worker's of the multi-device twins; the
+// caller holds g_cache_mu): pair buffers of one window of W pairs.
+static int window_plan(icikt_plan*& slot, int64_t n, int64_t C, int64_t W, const icikt_opts& o, icikt_plan** out) {
+  icikt_plan* p = slot;
   if (p && p->n == n && p->C == C && p->P == W && p->opts.device == o.device && p->opts.include_diag == o.include_diag) {
     p->opts.perspective = o.perspective;
     p->opts.alternative = o.alternative;
@@ -2058,22 +2150,22 @@ static int window_plan(int64_t n, int64_t C, int64_t W, const icikt_opts& o, ici
     p->opts.na_inf = o.na_inf;
   } else {
     if (p) icikt_plan_destroy(p);
-    g_cached_edges = nullptr;
+    slot = nullptr;
     icikt_opts po = o;
     po.pair_hi = W;  // the plan's pair buffers: one window
     const int rc = plan_create_impl(&p, n, C, nullptr, nullptr, 0, &po, false);
     if (rc != ICIKT_OK) return rc;
-    g_cached_edges = p;
+    slot = p;
   }
   *out = p;
   return ICIKT_OK;
 }
 
 // after a failed call: the cached plan goes, keeping the call's error message
-static void drop_window_plan() {
+static void drop_window_plan(icikt_plan*& slot) {
   const std::string keep = g_err;
-  icikt_plan_destroy(g_cached_edges);  // waits for whatever the failed call left in flight
-  g_cached_edges = nullptr;
+  icikt_plan_destroy(slot);  // waits for whatever the failed call left in flight
+  slot = nullptr;
   g_err = keep;
 }
 
@@ -2098,10 +2190,10 @@ static int all_pairs_edges(const ColumnSource& s, int64_t n, int64_t C, const do
   const int64_t W = std::min(edge_window(), ptot);
   std::lock_guard<std::mutex> lock(g_cache_mu);
   icikt_plan* p = nullptr;
-  rc = window_plan(n, C, W, o, &p);
+  rc = window_plan(g_cached_edges, n, C, W, o, &p);
   if (rc == ICIKT_OK) rc = edge_windows(p, s, global_na, n_global_na, *filter, ptot, W, res, max_taumax, timings);
   if (rc != ICIKT_OK) {
-    drop_window_plan();
+    drop_window_plan(g_cached_edges);
     delete res;
     return rc;
   }
@@ -2133,10 +2225,10 @@ static int all_pairs_topk(const ColumnSource& s, int64_t n, int64_t C, const dou
   const int64_t W = std::min(edge_window(), ptot);
   std::lock_guard<std::mutex> lock(g_cache_mu);
   icikt_plan* p = nullptr;
-  rc = window_plan(n, C, W, o, &p);
+  rc = window_plan(g_cached_edges, n, C, W, o, &p);
   if (rc == ICIKT_OK)
     rc = topk_windows(p, s, global_na, n_global_na, k, by, scale_max != 0, ptot, W, out, max_taumax, timings);
-  if (rc != ICIKT_OK) drop_window_plan();
+  if (rc != ICIKT_OK) drop_window_plan(g_cached_edges);
   return rc;
 }
 
@@ -2361,8 +2453,50 @@ int enable_peers(const MultiJob& J, int k) {
   return ICIKT_OK;
 }
 
-// Worker k up to and including the pair kernel + epilogue (results stay on its device).  In gather mode
-// every worker passes both barriers whatever happened to it, so nobody is left waiting.
+// The column phase of worker k on its plan p (rc: how getting the plan went): sharded K1 and the peer gather of the
+// tables in gather mode, otherwise the upload and K1 of all columns (skipped when the worker has no pairs).  In
+// gather mode every worker passes both barriers whatever happened to it, so nobody is left waiting.
+int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
+  const int64_t cnt = J.pair_lo(k + 1) - J.pair_lo(k);
+  if (!J.gather) {
+    if (cnt <= 0) return rc;
+    if (rc == ICIKT_OK) rc = J.src.csc() ? upload_columns(p, J.src, 0, J.C) : icikt_plan_upload(p, J.src.data, J.src.ld);
+    if (rc == ICIKT_OK) rc = icikt_plan_columns(p, J.global_na, J.n_global_na);
+    return rc;
+  }
+  if (rc == ICIKT_OK) rc = upload_columns(p, J.src, J.col_lo(k), J.col_lo(k + 1));
+  if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
+  if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "column slice");
+  J.peer_plan[(size_t)k] = (rc == ICIKT_OK) ? p : nullptr;
+  J.barrier.wait();  // every slice of the tables is complete on its device
+  bool all_ok = true;
+  for (int j = 0; j < J.n_devices; ++j) all_ok = all_ok && J.peer_plan[(size_t)j] != nullptr;
+  if (rc == ICIKT_OK && !all_ok) rc = fail(ICIKT_ERR_CUDA, "a peer device failed to preprocess its slice");
+  if (rc == ICIKT_OK) rc = enable_peers(J, k);
+  if (rc == ICIKT_OK) {
+    const int dev = J.device_of(k);
+    icikt_table mine[ICIKT_MAX_TABLES], theirs[ICIKT_MAX_TABLES];
+    const int nt = icikt_plan_tables(p, mine, ICIKT_MAX_TABLES);
+    for (int j = 0; j < J.n_devices && rc == ICIKT_OK; ++j) {
+      if (j == k) continue;
+      icikt_plan_tables(J.peer_plan[(size_t)j], theirs, ICIKT_MAX_TABLES);
+      for (int t = 0; t < nt && rc == ICIKT_OK; ++t) {
+        const size_t off = (size_t)J.col_lo(j) * (size_t)mine[t].bytes_per_column;
+        const size_t len = (size_t)(J.col_lo(j + 1) - J.col_lo(j)) * (size_t)mine[t].bytes_per_column;
+        if (len && cudaMemcpyPeerAsync(static_cast<unsigned char*>(mine[t].ptr) + off, dev,
+                                       static_cast<const unsigned char*>(theirs[t].ptr) + off, J.device_of(j), len,
+                                       p->stream) != cudaSuccess)
+          rc = cuda_fail(cudaGetLastError(), "cudaMemcpyPeerAsync");
+      }
+    }
+    if (rc == ICIKT_OK) rc = icikt_plan_columns_finish(p);
+    if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "peer gather");
+  }
+  J.barrier.wait();  // nobody's tables are touched (or freed) before every pull has finished
+  return rc;
+}
+
+// Worker k up to and including the pair kernel + epilogue (results stay on its device).
 int multi_worker_pairs(MultiJob& J, int k, icikt_plan** out) {
   int rc = ICIKT_OK;
   icikt_opts o = J.base;
@@ -2386,42 +2520,8 @@ int multi_worker_pairs(MultiJob& J, int k, icikt_plan** out) {
     if (rc == ICIKT_OK) slot = p;
   }
   *out = p;
-  if (!J.gather) {
-    if (cnt <= 0) return rc;
-    if (rc == ICIKT_OK) rc = J.src.csc() ? upload_columns(p, J.src, 0, J.C) : icikt_plan_upload(p, J.src.data, J.src.ld);
-    if (rc == ICIKT_OK) rc = icikt_plan_columns(p, J.global_na, J.n_global_na);
-  } else {
-    if (rc == ICIKT_OK) rc = upload_columns(p, J.src, J.col_lo(k), J.col_lo(k + 1));
-    if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
-    if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "column slice");
-    J.peer_plan[(size_t)k] = (rc == ICIKT_OK) ? p : nullptr;
-    J.barrier.wait();  // every slice of the tables is complete on its device
-    bool all_ok = true;
-    for (int j = 0; j < J.n_devices; ++j) all_ok = all_ok && J.peer_plan[(size_t)j] != nullptr;
-    if (rc == ICIKT_OK && !all_ok) rc = fail(ICIKT_ERR_CUDA, "a peer device failed to preprocess its slice");
-    if (rc == ICIKT_OK) rc = enable_peers(J, k);
-    if (rc == ICIKT_OK) {
-      icikt_table mine[ICIKT_MAX_TABLES], theirs[ICIKT_MAX_TABLES];
-      const int nt = icikt_plan_tables(p, mine, ICIKT_MAX_TABLES);
-      for (int j = 0; j < J.n_devices && rc == ICIKT_OK; ++j) {
-        if (j == k) continue;
-        icikt_plan_tables(J.peer_plan[(size_t)j], theirs, ICIKT_MAX_TABLES);
-        for (int t = 0; t < nt && rc == ICIKT_OK; ++t) {
-          const size_t off = (size_t)J.col_lo(j) * (size_t)mine[t].bytes_per_column;
-          const size_t len = (size_t)(J.col_lo(j + 1) - J.col_lo(j)) * (size_t)mine[t].bytes_per_column;
-          if (len && cudaMemcpyPeerAsync(static_cast<unsigned char*>(mine[t].ptr) + off, o.device,
-                                         static_cast<const unsigned char*>(theirs[t].ptr) + off, J.device_of(j), len,
-                                         p->stream) != cudaSuccess)
-            rc = cuda_fail(cudaGetLastError(), "cudaMemcpyPeerAsync");
-        }
-      }
-      if (rc == ICIKT_OK) rc = icikt_plan_columns_finish(p);
-      if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "peer gather");
-    }
-    J.barrier.wait();  // nobody's tables are touched (or freed) before every pull has finished
-    if (cnt <= 0) return rc;
-  }
-  if (rc == ICIKT_OK) rc = icikt_plan_pairs(p);
+  rc = multi_worker_columns(J, k, p, rc);
+  if (rc == ICIKT_OK && cnt > 0) rc = icikt_plan_pairs(p);
   return rc;
 }
 
@@ -2626,6 +2726,220 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
   return ICIKT_OK;
 }
 
+// ---- the filtered calls over several devices: the pair order sliced as in icikt_all_pairs_multi, every slice
+// walked window by window on its device, the per-device results combined exactly
+
+int check_window_devices(int32_t n_devices) {
+  if (n_devices < 1 || n_devices > kMaxMatrixDevices) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..16");
+  return ICIKT_OK;
+}
+
+// Worker k of a filtered multi-device call up to its window walk: its window plan (cached per worker slot, windows of
+// min(ICIKT_EDGE_WINDOW, its slice) pairs and at least one) and the column phase.
+int window_multi_worker(MultiJob& J, int k, icikt_plan** out) {
+  icikt_opts o = J.base;
+  o.device = J.device_of(k);
+  const int64_t W = std::max<int64_t>(1, std::min(edge_window(), J.pair_lo(k + 1) - J.pair_lo(k)));
+  icikt_plan* p = nullptr;
+  int rc = window_plan(g_cached_wmulti[k], J.n, J.C, W, o, &p);
+  *out = p;
+  rc = multi_worker_columns(J, k, p, rc);
+  if (rc == ICIKT_OK) CK(cudaSetDevice(p->device));
+  return rc;
+}
+
+int edges_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                     const icikt_opts* opts, const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
+                     icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  int rc = check_edge_args(s, n, C, global_na, n_global_na, o, filter, out);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t ptot = tri_pairs(C) + (o.include_diag ? C : 0);
+  MultiJob J(n_devices);
+  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.ptot = ptot;
+  if (n_devices == 1 || ptot == 0) {
+    o.device = J.device_of(0);
+    return all_pairs_edges(s, n, C, global_na, n_global_na, &o, filter, out, max_taumax, timings);
+  }
+  rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
+  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
+  const icikt_edge_filter& f = *filter;
+  std::vector<MultiWork> work((size_t)n_devices);
+  std::vector<std::vector<EdgeRow>> rows((size_t)n_devices);
+  std::vector<unsigned long long> bits((size_t)n_devices, 0);
+  EdgeHeld held;
+  {
+    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+    multi_probe_peers(J);
+    std::vector<std::thread> threads;
+    for (int k = 0; k < n_devices; ++k) {
+      threads.emplace_back([&, k]() {
+        MultiWork& w = work[(size_t)k];
+        icikt_plan* p = nullptr;
+        w.rc = window_multi_worker(J, k, &p);
+        const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
+        if (w.rc == ICIKT_OK && hi > lo) {
+          WalkTotals tot;
+          float d2h_ms = 0.f;
+          w.rc = ensure_edge_buffers(p, p->P);
+          if (w.rc == ICIKT_OK) w.rc = edge_walk(p, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
+          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
+          bits[(size_t)k] = tot.bits;
+        }
+        if (w.rc != ICIKT_OK) {
+          w.err = g_err;  // thread-local message of this worker
+          drop_window_plan(g_cached_wmulti[k]);
+        }
+      });
+    }
+    for (auto& t : threads) t.join();
+  }
+  rc = multi_collect(work, nullptr, timings);
+  if (rc != ICIKT_OK) return rc;
+  // the slices are contiguous and in worker order: so are the rows
+  size_t total = 0;
+  for (const auto& r : rows) total += r.size();
+  try {
+    res->rows.reserve(total);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the selected rows");
+  }
+  for (auto& r : rows) {
+    res->rows.insert(res->rows.end(), r.begin(), r.end());
+    std::vector<EdgeRow>().swap(r);
+  }
+  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  rc = edge_result(res.get(), f, M);
+  if (rc != ICIKT_OK) return rc;
+  if (max_taumax) *max_taumax = M;
+  *out = res.release();
+  return ICIKT_OK;
+}
+
+// Worker k's block of columns [col_lo(k), col_lo(k + 1)) of the merged lists: the merge kernel reads every device's
+// lists in place, and the block goes straight into the caller's arrays at c_lo * k (raw: out.raw or the host
+// buffer for cor); held[c] receives column c's entries.  tm: the merge and its copies become d2h_ms.
+int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<icikt_plan*>& plans, int K, int by,
+                     const TopkOut& out, double* raw, int32_t* held, icikt_timings& tm) {
+  const int64_t c_lo = J.col_lo(k), c_hi = J.col_lo(k + 1);
+  if (c_hi <= c_lo) return ICIKT_OK;
+  const size_t blk = (size_t)(c_hi - c_lo) * (size_t)K, off = (size_t)c_lo * (size_t)K;
+  int rc = ensure_merge_buffers(p, blk);
+  if (rc != ICIKT_OK) return rc;
+  TopkDeviceMerge m{};
+  m.n_dev = J.n_devices;
+  for (int j = 0; j < J.n_devices; ++j) {
+    m.col[j] = plans[(size_t)j]->d_tcol;
+    m.idx[j] = plans[(size_t)j]->d_tidx;
+    m.list[j] = plans[(size_t)j]->d_tlist;
+  }
+  m.C = J.C;
+  m.c_lo = c_lo;
+  m.c_hi = c_hi;
+  m.k = K;
+  m.by = by;
+  m.n = p->d_mn;
+  m.out_idx = p->d_midx;
+  m.out = p->d_mlist;
+  CK(cudaEventRecord(p->ev[6], p->stream));
+  const int l = launch_topk_device_merge(m, p->stream);
+  if (l < 0) return launch_fail("top-k device merge kernel");
+  tm.n_launches += l;
+  rc = staged_copy_out(p, held + c_lo, p->d_mn, sizeof(int32_t) * (size_t)(c_hi - c_lo), p->stream);
+  if (rc == ICIKT_OK) rc = staged_copy_out(p, out.index + off, p->d_midx, sizeof(int32_t) * blk, p->stream);
+  double* host_field[4] = {raw, out.pvalue, out.taumax, out.completeness};
+  for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
+    if (host_field[f]) rc = staged_copy_out(p, host_field[f] + off, p->d_mlist + f * blk, sizeof(double) * blk, p->stream);
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[7], p->stream));
+  CK(cudaEventSynchronize(p->ev[7]));
+  tm.d2h_ms = ev_ms(p->ev[6], p->ev[7]);
+  tm.total_ms = ev_ms(p->ev[0], p->ev[7]);
+  cudaGetLastError();
+  return ICIKT_OK;
+}
+
+int topk_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                    const icikt_opts* opts, const int32_t* devices, int32_t n_devices, int32_t K, int32_t by,
+                    int32_t scale_max, const TopkOut& out, double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  int rc = check_topk_args(s, n, C, global_na, n_global_na, o, K, by, out.index);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t ptot = tri_pairs(C);
+  MultiJob J(n_devices);
+  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.ptot = ptot;
+  rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  {
+    std::lock_guard<std::mutex> lock(g_cache_mu);
+    multi_probe_peers(J);
+  }
+  if (n_devices == 1 || !J.peers_ok || ptot == 0) {
+    // one device, or devices that cannot read each other's lists: the single-device call
+    o.device = J.device_of(0);
+    return all_pairs_topk(s, n, C, global_na, n_global_na, &o, K, by, scale_max, out, max_taumax, timings);
+  }
+  const int64_t ck = C * K;
+  std::vector<double> raw_own;
+  double* raw = nullptr;
+  rc = topk_raw_buffer(out, ck, raw_own, &raw);
+  if (rc != ICIKT_OK) return rc;
+  std::vector<int32_t> held;
+  try {
+    held.resize((size_t)C);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
+  }
+  std::vector<MultiWork> work((size_t)n_devices);
+  std::vector<unsigned long long> bits((size_t)n_devices, 0);
+  std::vector<icikt_plan*> plans((size_t)n_devices, nullptr);
+  {
+    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+    std::vector<std::thread> threads;
+    for (int k = 0; k < n_devices; ++k) {
+      threads.emplace_back([&, k]() {
+        MultiWork& w = work[(size_t)k];
+        icikt_plan* p = nullptr;
+        w.rc = window_multi_worker(J, k, &p);
+        if (w.rc == ICIKT_OK) {
+          WalkTotals tot;
+          w.rc = ensure_topk_buffers(p, p->P, K);
+          if (w.rc == ICIKT_OK) w.rc = topk_walk(p, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
+          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, 0.f, &w.tm);
+          bits[(size_t)k] = tot.bits;
+        }
+        plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
+        J.barrier.wait();  // every device's lists are complete
+        bool all_ok = true;
+        for (int j = 0; j < n_devices; ++j) all_ok = all_ok && plans[(size_t)j] != nullptr;
+        if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to select its lists");
+        if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
+        if (w.rc == ICIKT_OK) w.rc = topk_merge_block(J, k, p, plans, K, by, out, raw, held.data(), w.tm);
+        J.barrier.wait();  // nobody's lists are freed (or reused) before every block has been merged
+        if (w.rc != ICIKT_OK) {
+          w.err = g_err;
+          drop_window_plan(g_cached_wmulti[k]);
+        }
+      });
+    }
+    for (auto& t : threads) t.join();
+  }
+  rc = multi_collect(work, nullptr, timings);
+  if (rc != ICIKT_OK) return rc;
+  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  topk_fill_host(out, C, K, [&](int64_t c) { return (int64_t)held[(size_t)c]; }, raw, scale_max != 0, M);
+  if (max_taumax) *max_taumax = M;
+  return ICIKT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2671,6 +2985,47 @@ int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const
   return matrices_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices,
                              n_devices, scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness,
                              status_counts, max_taumax, timings);
+}
+
+int icikt_all_pairs_edges_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                                int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                                icikt_timings* timings) {
+  return edges_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, filter, out,
+                          max_taumax, timings);
+}
+
+int icikt_all_pairs_edges_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                                    int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                                    const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
+                                    icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  if (out) *out = nullptr;
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return edges_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices, n_devices,
+                          filter, out, max_taumax, timings);
+}
+
+int icikt_all_pairs_topk_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                               int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                               int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
+                               double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                               double* max_taumax, icikt_timings* timings) {
+  return topk_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, k, by,
+                         scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax,
+                         timings);
+}
+
+int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                                   int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                                   const int32_t* devices, int32_t n_devices, int32_t k, int32_t by, int32_t scale_max,
+                                   int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
+                                   double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  return topk_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices, n_devices, k,
+                         by, scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness},
+                         max_taumax, timings);
 }
 
 int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,

@@ -251,6 +251,22 @@ struct TopkSelect {
 };
 int launch_topk_select(const TopkSelect& s, cudaStream_t stream);
 
+// The top-k call over several devices (icikt_all_pairs_topk_multi): every device holds the lists of its slice of
+// the pair order; one CTA per column of [c_lo, c_hi) folds the devices' lists into one, reading them through peer
+// pointers, and gathers the kept entries' fields from the device that holds them.
+struct TopkDeviceMerge {
+  int n_dev;  // <= kMaxMatrixDevices
+  const TopkCol* col[kMaxMatrixDevices];   // [C] each
+  const int32_t* idx[kMaxMatrixDevices];   // [C k] each
+  const double* list[kMaxMatrixDevices];   // 4 x [C k] each: raw, pvalue, taumax, completeness
+  long long C, c_lo, c_hi;
+  int k, by;
+  int32_t* n;     // this device's block: [c_hi - c_lo] entries kept
+  int32_t* out_idx;  // [(c_hi - c_lo) k]
+  double* out;    // 4 x [(c_hi - c_lo) k]: raw, pvalue, taumax, completeness
+};
+int launch_topk_device_merge(const TopkDeviceMerge& m, cudaStream_t stream);
+
 int launch_pnorm(const double* d_z, int64_t n, int lower, double* d_out, cudaStream_t stream);
 
 int64_t tiled_max_n();

@@ -9,7 +9,8 @@
 // HBM-bound: the count pass reads the status and, only for a bound that is given, raw (8 B) and the p-value
 // (8 B); the scatter pass reads 1/8 B of mask per slot and the fields of the kept slots.
 // The selection of the top-k call (icikt_all_pairs_topk) follows the edge kernels: per-column buckets of the
-// candidates that beat a column's k-th entry, merged into the column's sorted list (see launch_topk_select).
+// candidates that beat a column's k-th entry, merged into the column's sorted list (see launch_topk_select).  Over
+// several devices, topk_device_merge_kernel folds the devices' lists of a block of columns into one.
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
 #include "icikt_topk.cuh"
@@ -311,7 +312,77 @@ __global__ void __launch_bounds__(kMergeThreads) topk_merge_kernel(const TopkSel
   }
 }
 
+// One CTA per column of the block, one thread per list position.  The devices' lists fold one at a time into the
+// shared accumulator (at most k entries, best first) by merge path: an entry's new position is its index in its own
+// list plus its rank in the other (topk_rank), and entries that land at k or beyond drop out.  Partners are disjoint
+// across devices, so the positions are distinct.  Each kept entry remembers (device, position) and its fields are
+// read from that device once, after the last fold.
+__global__ void __launch_bounds__(kTopkMax) topk_device_merge_kernel(const TopkDeviceMerge m) {
+  __shared__ unsigned long long akey[kTopkMax], bkey[kTopkMax];
+  __shared__ int32_t apart[kTopkMax], bpart[kTopkMax];
+  __shared__ int32_t asrc[kTopkMax];  // device * kTopkMax + position in that device's list
+  const long long c = m.c_lo + blockIdx.x;
+  const int k = m.k, tid = threadIdx.x;
+  const long long base = c * k;
+  int a = 0;
+  for (int d = 0; d < m.n_dev; ++d) {
+    const int b = m.col[d][c].n;
+    if (b == 0) continue;
+    if (tid < b) {
+      bkey[tid] = topk_key(m.list[d][base + tid], m.by);
+      bpart[tid] = m.idx[d][base + tid];
+    }
+    __syncthreads();
+    int pa = k, pb = k;
+    unsigned long long ka = 0ull;
+    int32_t ia = 0, sa = 0;
+    if (tid < a) {
+      ka = akey[tid];
+      ia = apart[tid];
+      sa = asrc[tid];
+      pa = tid + topk_rank(bkey, bpart, b, ka, ia);
+    }
+    if (tid < b) pb = tid + topk_rank(akey, apart, a, bkey[tid], bpart[tid]);
+    const unsigned long long kb = tid < b ? bkey[tid] : 0ull;
+    const int32_t ib = tid < b ? bpart[tid] : 0;
+    __syncthreads();
+    if (pa < k) {
+      akey[pa] = ka;
+      apart[pa] = ia;
+      asrc[pa] = sa;
+    }
+    if (pb < k) {
+      akey[pb] = kb;
+      apart[pb] = ib;
+      asrc[pb] = d * kTopkMax + tid;
+    }
+    a = min(a + b, k);
+    __syncthreads();
+  }
+  const long long ck = m.C * k, blk = (m.c_hi - m.c_lo) * k, o = blockIdx.x * (long long)k + tid;
+  if (tid < a) {
+    const int d = asrc[tid] / kTopkMax;
+    const long long q = base + asrc[tid] % kTopkMax;
+    const double* l = m.list[d];
+    m.out_idx[o] = apart[tid];
+    m.out[o] = l[q];
+    m.out[blk + o] = l[ck + q];
+    m.out[2 * blk + o] = l[2 * ck + q];
+    m.out[3 * blk + o] = l[3 * ck + q];
+  }
+  if (tid == 0) m.n[blockIdx.x] = a;
+}
+
 }  // namespace
+
+int launch_topk_device_merge(const TopkDeviceMerge& m, cudaStream_t stream) {
+  if (m.c_hi <= m.c_lo) return launch_status(0);
+  if (m.n_dev < 1 || m.n_dev > kMaxMatrixDevices || m.k < 1 || m.k > kTopkMax || m.c_hi - m.c_lo > 0x7fffffffLL)
+    return launch_refused("top-k device merge: bad arguments");
+  const int threads = (m.k + 31) / 32 * 32;
+  topk_device_merge_kernel<<<(unsigned)(m.c_hi - m.c_lo), threads, 0, stream>>>(m);
+  return launch_status(1);
+}
 
 int launch_topk_select(const TopkSelect& s, cudaStream_t stream) {
   if (s.n_slots <= 0) return launch_status(0);

@@ -1,5 +1,6 @@
 // icikt_topk.cuh -- the ranking of the top-k all-pairs call (icikt_all_pairs_topk).  __host__ __device__ so that
-// the selection kernels and the tests (tests/topk_host.cpp, compiled by g++) run the same code.
+// the selection kernels and the tests (tests/topk_host.cpp, tests/topk_merge_host.cpp, compiled by g++) run the
+// same code.
 //
 // A candidate of column c is a partner d with its pair's raw.  Candidates are ranked by (key descending,
 // partner ascending), a strict total order since a partner occurs once per column.  The key is a uint64 whose
@@ -22,6 +23,18 @@ ICIKT_HD unsigned long long topk_key(double raw, int by) {
 // does (ka, ia) come before (kb, ib)?
 ICIKT_HD bool topk_before(unsigned long long ka, int32_t ia, unsigned long long kb, int32_t ib) {
   return ka > kb || (ka == kb && ia < ib);
+}
+
+// The merge-path rank of the device merge (icikt_all_pairs_topk_multi): how many entries of the sorted list
+// (key, part)[0..m) come before (k0, p0).  Merging two sorted lists whose partners are disjoint, an entry lands at
+// its index in its own list plus its rank in the other one; the positions are distinct since the order is strict.
+ICIKT_HD int topk_rank(const unsigned long long* key, const int32_t* part, int m, unsigned long long k0, int32_t p0) {
+  int lo = 0, hi = m;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (topk_before(key[mid], part[mid], k0, p0)) lo = mid + 1; else hi = mid;
+  }
+  return lo;
 }
 
 }  // namespace icikt

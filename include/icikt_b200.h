@@ -312,6 +312,47 @@ int icikt_all_pairs_topk_csc(const int64_t* colptr, const int32_t* rowidx, const
                              double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
                              double* max_taumax, icikt_timings* timings);
 
+/* ---- the filtered and the top-k all-pairs calls over several GPUs of one box in ONE call.  The pair order is sliced
+ * over the devices as in icikt_all_pairs_multi (sharded K1 + peer gather of the tables when every pair of devices has
+ * peer access, otherwise every device preprocesses all columns), and device k walks its slice in windows of
+ * min(ICIKT_EDGE_WINDOW, slice) pairs.  Edges: every device keeps the rows of its slice against its own running
+ * maximum (a superset of the final rows); the host trims them with the final maximum M over all devices and joins
+ * them in slice order.  Top-k: every device keeps the lists of its slice; then device k merges the lists of all
+ * devices for columns [C*k/N, C*(k+1)/N), reading them in place through peer access, and copies its block straight
+ * into the caller's arrays.  Without peer access between distinct devices, or with one device, the top-k call runs
+ * icikt_all_pairs_topk on devices[0]; the edges call runs icikt_all_pairs_edges there with one device.
+ *
+ *   - Same result as one device: every output (rows, their order and fields, cor, max_taumax, index, n_neighbors,
+ *     the padding, what icikt_edges_copy returns) is bit for bit that of the single-device call.
+ *   - devices == NULL means ordinals 0..n_devices-1; repeated ordinals are allowed; 1 <= n_devices <= 16.
+ *     opts->device is ignored.
+ *   - Refused with ICIKT_ERR_BAD_ARG before any device is touched: whatever the single-device call refuses, and
+ *     n_devices out of range.
+ *   - max_edges counts the rows held over all devices.  Without scale_max or without min_abs_cor the call fails with
+ *     ICIKT_ERR_LIMIT exactly when more than max_edges pairs pass; with both, the held count may include rows the
+ *     final maximum removes, as in the single-device call.  When one device crosses the limit, the others stop at
+ *     their next window boundary.
+ *   - timings (may be NULL): the slowest device's figures, n_launches summed over the devices; for top-k, d2h_ms is
+ *     the merge of the device's block with its copy out. */
+int icikt_all_pairs_edges_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                                int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                                icikt_timings* timings);
+int icikt_all_pairs_edges_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                                    int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                                    const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
+                                    icikt_edges** out, double* max_taumax, icikt_timings* timings);
+int icikt_all_pairs_topk_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                               int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                               int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
+                               double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                               double* max_taumax, icikt_timings* timings);
+int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                                   int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                                   const int32_t* devices, int32_t n_devices, int32_t k, int32_t by, int32_t scale_max,
+                                   int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
+                                   double* taumax, double* completeness, double* max_taumax, icikt_timings* timings);
+
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
  * pay the copies.  A plan is bound to one device and is not thread-safe.            */
