@@ -40,7 +40,7 @@ EXPORTS = [
     "icikt_all_pairs_edges", "icikt_all_pairs_edges_csc", "icikt_edges_count", "icikt_edges_copy",
     "icikt_edges_free", "icikt_all_pairs_topk", "icikt_all_pairs_topk_csc",
     "icikt_all_pairs_edges_multi", "icikt_all_pairs_edges_multi_csc", "icikt_all_pairs_topk_multi",
-    "icikt_all_pairs_topk_multi_csc",
+    "icikt_all_pairs_topk_multi_csc", "icikt_cross_pairs", "icikt_cross_edges", "icikt_cross_topk",
 ]
 NSTATUS = 10
 
@@ -74,6 +74,19 @@ class Timings(ctypes.Structure):
 class EdgeFilter(ctypes.Structure):
     _fields_ = [("min_abs_cor", ctypes.c_double), ("max_pvalue", ctypes.c_double),
                 ("scale_max", ctypes.c_int32), ("reserved", ctypes.c_int32), ("max_edges", ctypes.c_int64)]
+
+
+class Input(ctypes.Structure):
+    """icikt_input: one matrix of a cross call, dense (data, ld) or CSC (colptr, rowidx, values)."""
+    _fields_ = [("C", ctypes.c_int64), ("data", ctypes.c_void_p), ("ld", ctypes.c_int64),
+                ("colptr", ctypes.c_void_p), ("rowidx", ctypes.c_void_p), ("values", ctypes.c_void_p)]
+
+
+class TopkLists(ctypes.Structure):
+    """icikt_topk_lists: the caller arrays of one side of icikt_cross_topk."""
+    _fields_ = [("index", ctypes.c_void_p), ("n_neighbors", ctypes.c_void_p), ("cor", ctypes.c_void_p),
+                ("raw", ctypes.c_void_p), ("pvalue", ctypes.c_void_p), ("taumax", ctypes.c_void_p),
+                ("completeness", ctypes.c_void_p)]
 
 
 class Table(ctypes.Structure):
@@ -187,6 +200,14 @@ def load():
             f = getattr(L, name + sfx)
             f.argtypes = lead + [_ip, ctypes.c_int32] + a[7:]
             f.restype = ctypes.c_int
+    cross = [ctypes.POINTER(Input), ctypes.POINTER(Input), ctypes.c_int64, _dp, ctypes.c_int32, ctypes.POINTER(Opts)]
+    L.icikt_cross_pairs.argtypes = cross + [_dp, _dp, _dp, _dp, _ip, _dp, ctypes.POINTER(Timings)]
+    L.icikt_cross_pairs.restype = ctypes.c_int
+    L.icikt_cross_edges.argtypes = cross + L.icikt_all_pairs_edges.argtypes[7:]
+    L.icikt_cross_edges.restype = ctypes.c_int
+    L.icikt_cross_topk.argtypes = cross + [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(TopkLists),
+                                           ctypes.POINTER(TopkLists), _dp, ctypes.POINTER(Timings)]
+    L.icikt_cross_topk.restype = ctypes.c_int
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -432,6 +453,111 @@ def run_topk(data, global_na=(), k=10, by="abs", scale_max=True, devices=None, *
                                                           _ptr(out["n_neighbors"]),
                                                           *(_ptr(out[name]) for name in EDGE_NAMES), ctypes.byref(mx),
                                                           ctypes.byref(t)))
+    out.update(max_taumax=mx.value, timings=t.as_dict())
+    return out
+
+
+def _cross_inputs(x, y):
+    """(icikt_input of x, of y, n, Cx, Cy, the objects that own the memory they point into) for the cross calls; x
+    and y may each be a NumPy array or a scipy.sparse matrix"""
+    ins, keep = [], []
+    for a in (x, y):
+        if is_sparse(a):
+            m = CSC(a)
+            ins.append(Input(m.shape[1], None, 0, _ptr(m.colptr), _ptr(m.rowidx), _ptr(m.values)))
+            shape = m.shape
+        else:
+            m = np.asfortranarray(a, dtype=np.float64)
+            if m.ndim != 2:
+                raise ValueError("x and y must be 2-D arrays (features x samples)")
+            ins.append(Input(m.shape[1], _ptr(m), m.shape[0], None, None, None))
+            shape = m.shape
+        keep.append((m, shape))
+    (_, (nx, cx)), (_, (ny, cy)) = keep
+    if nx != ny:
+        raise ValueError(f"x has {nx} rows and y has {ny}: the cross calls need the same rows")
+    return ins[0], ins[1], nx, cx, cy, keep
+
+
+def run_cross(x, y, global_na=(), **opt_kw):
+    """icikt_cross_pairs: every column of x against every column of y (same rows), pair p = i * Cy + j in x-major
+    order; pair_lo / pair_hi select a slice (0, 0: all).  Every field is bit for bit run_pairs(hstack([x, y]),
+    pi=i, pj=Cx + j)'s.  x and y may each be a NumPy array or a scipy.sparse matrix.  Returns a dict of NumPy arrays
+    in pair order: raw, pvalue, taumax, completeness, status, plus max_taumax and timings."""
+    L = load()
+    xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    o = make_opts(**opt_kw)
+    P = cx * cy if (o.pair_lo == 0 and o.pair_hi == 0) else max(o.pair_hi - o.pair_lo, 0)
+    buf = np.empty(4 * P + (P + 1) // 2, dtype=np.float64)
+    raw, pv, tm, comp = buf[:P], buf[P:2 * P], buf[2 * P:3 * P], buf[3 * P:4 * P]
+    status = buf[4 * P:].view(np.int32)[:P]
+    a = _ptr(buf)
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(L.icikt_cross_pairs(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o), a, a + 8 * P,
+                              a + 16 * P, a + 24 * P, a + 32 * P, ctypes.byref(mx), ctypes.byref(t)))
+    return dict(raw=raw, pvalue=pv, taumax=tm, completeness=comp, status=status, max_taumax=mx.value,
+                timings=t.as_dict())
+
+
+def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, **opt_kw):
+    """icikt_cross_edges: the pairs of x's columns with y's columns that pass the filter of run_edges, in cross
+    order, filtered on the device.  Returns the dict of run_edges; i indexes x's columns, j y's."""
+    L = load()
+    xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    o = make_opts(**opt_kw)
+    f = EdgeFilter(_bound(min_abs_cor), _bound(max_pvalue), int(bool(scale_max)), 0, int(max_edges))
+    h = ctypes.c_void_p()
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(L.icikt_cross_edges(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o), ctypes.byref(f),
+                              ctypes.byref(h), ctypes.byref(mx), ctypes.byref(t)))
+    try:
+        m = int(L.icikt_edges_count(h))
+        out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
+        out.update((k, np.empty(m, dtype=np.float64)) for k in EDGE_NAMES)
+        check(L.icikt_edges_copy(h, _ptr(out["i"]), _ptr(out["j"]), *(_ptr(out[k]) for k in EDGE_NAMES)))
+    finally:
+        L.icikt_edges_free(h)
+    out.update(max_taumax=mx.value, timings=t.as_dict())
+    return out
+
+
+CROSS_SIDES = {"x": (True, False), "y": (False, True), "both": (True, True)}
+
+
+def run_cross_topk(x, y, global_na=(), k=10, by="abs", scale_max=True, side="both", **opt_kw):
+    """icikt_cross_topk: each column's k best partners in the other matrix, in the order of run_topk.  side "x": the
+    lists of x's columns (partners are y indices), "y": of y's columns (partners are x indices), "both".  Returns a
+    dict with x_side and/or y_side (each the per-column arrays of run_topk: index, n_neighbors, cor, raw, pvalue,
+    taumax, completeness), max_taumax and timings."""
+    if by not in TOPK_BY:
+        raise ValueError(f"by must be one of {sorted(TOPK_BY)}")
+    if side not in CROSS_SIDES:
+        raise ValueError(f"side must be one of {sorted(CROSS_SIDES)}")
+    L = load()
+    xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    o = make_opts(**opt_kw)
+    k = int(k)
+    kk = k if 1 <= k <= TOPK_MAX else 0  # a k the library refuses gets no arrays
+    k = k if -2 ** 31 <= k < 2 ** 31 else 0  # and reaches it as a refused int32
+    out, lists = {}, []
+    for name, want, C in (("x_side", CROSS_SIDES[side][0], cx), ("y_side", CROSS_SIDES[side][1], cy)):
+        if not want:
+            lists.append(None)
+            continue
+        d = dict(index=np.empty((C, kk), dtype=np.int32), n_neighbors=np.empty(C, dtype=np.int32))
+        d.update((f, np.empty((C, kk), dtype=np.float64)) for f in EDGE_NAMES)
+        out[name] = d
+        lists.append(TopkLists(_ptr(d["index"]), _ptr(d["n_neighbors"]), *(_ptr(d[f]) for f in EDGE_NAMES)))
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(L.icikt_cross_topk(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o), k, TOPK_BY[by],
+                             int(bool(scale_max)), *(ctypes.byref(v) if v is not None else None for v in lists),
+                             ctypes.byref(mx), ctypes.byref(t)))
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 

@@ -404,6 +404,116 @@ def ici_kendalltau_topk(data_matrix, k, by="abs", global_na=(np.nan, np.inf, 0),
     return out
 
 
+def _cross_data(x, y, xnames, ynames):
+    x, xnames = _colnames_of(x, xnames, "x")
+    y, ynames = _colnames_of(y, ynames, "y")
+    if x.shape[0] != y.shape[0]:
+        raise ValueError(f"`x` has {x.shape[0]} rows and `y` has {y.shape[0]}: both need the same features")
+    return x, y, xnames, ynames
+
+
+def _names_by_index(names):
+    """names as an object array with a trailing None, which index -1 picks"""
+    nm = np.empty(len(names) + 1, dtype=object)
+    for c, v in enumerate(names):
+        nm[c] = v
+    return nm
+
+
+def ici_kendalltau_cross(x, y, global_na=(np.nan, np.inf, 0), perspective="global", scale_max=True,
+                         alternative="two.sided", continuity=False, return_matrix=True, min_abs_cor=None,
+                         max_pvalue=None, max_edges=None, xnames=None, ynames=None, device=0, n_gpus=1):
+    """ICI-Kendall-tau of every column (sample) of `x` with every column of `y`, both features x samples with the
+    same features: query samples against a reference panel, two batches, two feature sets on the same samples.
+
+    Every value is the one ici_kendalltau computes for that pair of columns side by side, with x's column first;
+    cor = raw / max(taumax over the Cx x Cy pairs) if scale_max else raw.  Returns a dict with `cor`, `raw`,
+    `pvalue`, `taumax`, `completeness` as (Cx, Cy) arrays (row i: x's column i), `xnames`, `ynames` and `run_time`;
+    with return_matrix=False a long table `cor` (dict of columns s1 from x, s2 from y, raw, pvalue, taumax,
+    completeness, cor) in x-major order.  The pairs run window by window on the device (_lib.run_cross), so device
+    memory does not grow with Cx x Cy.  Each degenerate class warns once.
+
+    min_abs_cor / max_pvalue (return_matrix=False) keep only the rows with abs(cor) >= min_abs_cor and
+    pvalue <= max_pvalue, selected on the device (_lib.run_cross_edges) with the rules of ici_kendalltau's filtered
+    table; max_edges raises IciktError (ERR_LIMIT) when more pairs pass.  One GPU: n_gpus must be 1.
+    """
+    if n_gpus != 1:
+        raise ValueError("the cross calls run on one GPU: n_gpus must be 1")
+    filtered = min_abs_cor is not None or max_pvalue is not None
+    if filtered and return_matrix:
+        raise ValueError("`min_abs_cor` and `max_pvalue` select rows of the long table: pass return_matrix=False")
+    if max_edges is not None and not filtered:
+        raise ValueError("`max_edges` limits a filtered table: give `min_abs_cor` or `max_pvalue` too")
+    x, y, xnames, ynames = _cross_data(x, y, xnames, ynames)
+    cx, cy = x.shape[1], y.shape[1]
+    global_na = [float(v) for v in global_na]
+    kw = dict(perspective=perspective, alternative=alternative, continuity=continuity, device=device)
+    log.info("Running correlations ...")
+    t1 = time.perf_counter()
+    if filtered:
+        r = _lib.run_cross_edges(x, y, global_na, min_abs_cor, max_pvalue, scale_max, max_edges or 0, **kw)
+        run_time = time.perf_counter() - t1
+        xn, yn = np.asarray(xnames, dtype=object), np.asarray(ynames, dtype=object)
+        return dict(cor=dict(s1=xn[r["i"]], s2=yn[r["j"]], raw=r["raw"], pvalue=r["pvalue"], taumax=r["taumax"],
+                             completeness=r["completeness"], cor=r["cor"]),
+                    run_time=run_time, xnames=xnames, ynames=ynames)
+    r = _lib.run_cross(x, y, global_na, **kw)
+    run_time = time.perf_counter() - t1
+    _warn_status(r["status"])
+    cols = {k: r[k] for k in ("raw", "pvalue", "taumax", "completeness")}
+    cols["cor"] = r["raw"] / r["max_taumax"] if scale_max else r["raw"].copy()
+    if not return_matrix:
+        xn, yn = np.asarray(xnames, dtype=object), np.asarray(ynames, dtype=object)
+        table = dict(s1=np.repeat(xn, cy), s2=np.tile(yn, cx))
+        table.update((k, cols[k]) for k in ("raw", "pvalue", "taumax", "completeness", "cor"))
+        return dict(cor=table, run_time=run_time, xnames=xnames, ynames=ynames)
+    out = {k: cols[k].reshape(cx, cy) for k in _lib.MATRIX_NAMES}
+    out.update(xnames=xnames, ynames=ynames, run_time=run_time)
+    return out
+
+
+def ici_kendalltau_cross_topk(x, y, k, by="abs", side="x", global_na=(np.nan, np.inf, 0), perspective="global",
+                              scale_max=True, alternative="two.sided", continuity=False, xnames=None, ynames=None,
+                              device=0, n_gpus=1):
+    """Each sample's k most correlated partners in the OTHER matrix (x and y: features x samples, same features).
+
+    side="x": for every column of x, its best columns of y (query against reference); "y": for every column of y,
+    its best columns of x; "both": the two lists, e.g. for mutual nearest neighbours between two batches.  Ranking,
+    padding and values are those of ici_kendalltau_topk over the Cx x Cy pairs; cor = raw / max(taumax over those
+    pairs) if scale_max else raw.  The lists are selected on the device window by window (_lib.run_cross_topk) and
+    held there only for the requested sides.  One GPU: n_gpus must be 1.
+
+    Returns a dict with key "x" and/or "y": per side the dict ici_kendalltau_topk returns (`index`, `neighbors` --
+    names from the other matrix --, `cor`, `raw`, `pvalue`, `taumax`, `completeness`, `n_neighbors`, `max_taumax`,
+    `run_time`, and `names`, the side's own column names).
+    """
+    if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.TOPK_MAX:
+        raise ValueError(f"`k` must be an integer in [1, {_lib.TOPK_MAX}], got {k!r}")
+    if by not in _lib.TOPK_BY:
+        raise ValueError(f"`by` must be 'abs' or 'signed', got {by!r}")
+    if side not in _lib.CROSS_SIDES:
+        raise ValueError(f"`side` must be 'x', 'y' or 'both', got {side!r}")
+    if n_gpus != 1:
+        raise ValueError("the cross calls run on one GPU: n_gpus must be 1")
+    x, y, xnames, ynames = _cross_data(x, y, xnames, ynames)
+    global_na = [float(v) for v in global_na]
+    log.info("Running correlations ...")
+    t1 = time.perf_counter()
+    r = _lib.run_cross_topk(x, y, global_na, int(k), by, scale_max, side, perspective=perspective,
+                            alternative=alternative, continuity=continuity, device=device)
+    run_time = time.perf_counter() - t1
+    out = {}
+    for key, own, other in (("x", xnames, ynames), ("y", ynames, xnames)):
+        if key + "_side" not in r:
+            continue
+        lists = r[key + "_side"]
+        d = {f: lists[f] for f in ("index", "cor", "raw", "pvalue", "taumax", "completeness", "n_neighbors")}
+        d["neighbors"] = _names_by_index(other)[lists["index"]]
+        d.update(max_taumax=r["max_taumax"], run_time=run_time, names=own)
+        out[key] = d
+    return out
+
+
 _NA_METHODS = ("all.obs", "complete.obs", "pairwise.complete.obs", "everything", "na.or.complete")
 
 

@@ -19,6 +19,7 @@
 #include <vector>
 
 #include "../../include/icikt_b200.h"
+#include "icikt_cross.cuh"
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
 #include "icikt_topk.cuh"
@@ -196,6 +197,7 @@ struct icikt_plan {
   double* d_values = nullptr;
   int64_t csc_cap = 0;                   // entries d_rowidx / d_values hold
   int64_t expand_lo = 0, expand_hi = 0;  // columns uploaded as CSC and not expanded yet
+  int64_t expand_dst = 0;                // ... and the matrix column their column 0 lands on (cross calls: Y at Cx)
 
   ColumnTables tab;
   ColumnWork wk;
@@ -259,13 +261,17 @@ struct icikt_plan {
   unsigned long long* h_estat = nullptr;   // pinned [2][2]: rows kept, max taumax bits so far
   cudaEvent_t eev[2][6]{};                 // per buffer: units up start/end, K2 start, K2 end, K3 end, selection end
   // Top-k all-pairs call (icikt_all_pairs_topk), on the same window walk: per-column candidate counts, the
-  // candidates of one window, and the lists of up to topk_cap entries per column
+  // candidates of one window, and the lists of the L columns that keep one (all C, or one side of a cross call)
   uint32_t* d_tcount = nullptr;
   uint2* d_tcand = nullptr;    // [2 W]
-  TopkCol* d_tcol = nullptr;   // [C]
-  int32_t* d_tidx = nullptr;   // [C k]
-  double* d_tlist = nullptr;   // 4 x [C k]: raw, pvalue, taumax, completeness
-  int topk_cap = 0;
+  TopkCol* d_tcol = nullptr;   // [L]
+  int32_t* d_tidx = nullptr;   // [L k]
+  double* d_tlist = nullptr;   // 4 x [L k]: raw, pvalue, taumax, completeness
+  int64_t topk_cols = 0;       // L d_tcount / d_tcol hold
+  int64_t topk_entries = 0;    // L k d_tidx / d_tlist hold
+  // Cross per-pair call (icikt_cross_pairs): a window's results, moved off the pair buffers so that they can be
+  // copied out while the next window runs; [tau W][pvalue W][taumax W][completeness W] doubles, [status W] int32
+  unsigned char* d_cres[2] = {nullptr, nullptr};
   // Top-k over several devices (icikt_all_pairs_topk_multi): this device's block of columns of the merged lists
   int32_t* d_mn = nullptr;     // [C] entries kept per column of the block
   int32_t* d_midx = nullptr;   // [merge_cap]
@@ -336,6 +342,8 @@ void free_plan(icikt_plan* p) {
   cudaFree(p->d_etotal);
   if (p->h_estat) cudaFreeHost(p->h_estat);
   cudaFree(p->d_tcount);
+  cudaFree(p->d_cres[0]);
+  cudaFree(p->d_cres[1]);
   cudaFree(p->d_tcand);
   cudaFree(p->d_tcol);
   cudaFree(p->d_tidx);
@@ -546,8 +554,9 @@ bool host_is_pinned(const void* ptr) {
 }
 
 // Where the columns of a call come from: a dense column-major matrix (data, ld) or a CSC matrix (colptr
-// [C + 1], rowidx / values [colptr[C]], checked by check_csc).
+// [C + 1], rowidx / values [colptr[C]], checked by check_csc) of C columns (icikt_input of the public header).
 struct ColumnSource {
+  int64_t C = 0;
   const double* data = nullptr;
   int64_t ld = 0;
   const int64_t* colptr = nullptr;
@@ -555,14 +564,16 @@ struct ColumnSource {
   const double* values = nullptr;
   bool csc() const { return colptr != nullptr; }
 };
-ColumnSource dense_source(const double* data, int64_t ld) {
+ColumnSource dense_source(const double* data, int64_t ld, int64_t C) {
   ColumnSource s;
+  s.C = C;
   s.data = data;
   s.ld = ld;
   return s;
 }
-ColumnSource csc_source(const int64_t* colptr, const int32_t* rowidx, const double* values) {
+ColumnSource csc_source(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t C) {
   ColumnSource s;
+  s.C = C;
   s.colptr = colptr;
   s.rowidx = rowidx;
   s.values = values;
@@ -642,11 +653,12 @@ int copy_array_in(icikt_plan* p, void* d_dst, const void* src, size_t bytes, cud
 }
 
 // CSC columns [c_lo, c_hi): the colptr slice and the slices [colptr[c_lo], colptr[c_hi]) of rowidx and values,
-// on `stream`.  The columns are expanded into d_data_own by the next plan_columns_impl, on the compute stream.
+// on `stream`.  The columns are expanded into d_data_own (source column c at matrix column dst + c) by the next
+// plan_columns_impl or expand_columns, on the compute stream.
 // (Neighbouring chunks of a pipelined call both copy their shared colptr entry; the second copy writes the
 // value the expansion of the first chunk may be reading.)
-int copy_csc_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, cudaStream_t stream) {
-  const int64_t nnz = s.colptr[p->C];
+int copy_csc_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, int64_t dst, cudaStream_t stream) {
+  const int64_t nnz = s.colptr[s.C];
   if (!p->d_colptr) CK(dmalloc(&p->d_colptr, (size_t)p->C + 1));
   if (nnz > p->csc_cap) {  // nothing of an earlier call is in flight: every call ends with its streams idle
     cudaFree(p->d_rowidx);
@@ -669,22 +681,25 @@ int copy_csc_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi
   if (rc != ICIKT_OK) return rc;
   p->expand_lo = c_lo;
   p->expand_hi = c_hi;
+  p->expand_dst = dst;
   return ICIKT_OK;
 }
 
-// host -> device copy of columns [c_lo, c_hi) into the plan's own matrix buffer (CSC: of their stored
-// entries), on `stream`
-int copy_columns_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, cudaStream_t stream) {
+// host -> device copy of columns [c_lo, c_hi) of `s` into the plan's own matrix buffer at matrix columns
+// [dst + c_lo, dst + c_hi) (CSC: of their stored entries), on `stream`
+int copy_columns_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, cudaStream_t stream,
+                    int64_t dst = 0) {
   if (!p->d_data_own) CK(dmalloc(&p->d_data_own, (size_t)p->n * p->C));
-  if (s.csc()) return copy_csc_in(p, s, c_lo, c_hi, stream);
+  if (s.csc()) return copy_csc_in(p, s, c_lo, c_hi, dst, stream);
   p->expand_lo = p->expand_hi = 0;
   const double* data = s.data;
   const int64_t ld = s.ld;
   if (c_hi <= c_lo) return ICIKT_OK;
+  double* out = p->d_data_own + (size_t)(dst + c_lo) * p->n;
   const size_t bytes = sizeof(double) * (size_t)p->n * (size_t)(c_hi - c_lo);
   if (ld == p->n && bytes >= (8u << 20) && !std::getenv("ICIKT_NO_STAGED_UPLOAD") && !host_is_pinned(data + (size_t)c_lo * ld))
-    return staged_copy_in(p, p->d_data_own + (size_t)c_lo * p->n, data + (size_t)c_lo * ld, bytes, stream);
-  CK(cudaMemcpy2DAsync(p->d_data_own + (size_t)c_lo * p->n, sizeof(double) * p->n, data + (size_t)c_lo * ld,
+    return staged_copy_in(p, out, data + (size_t)c_lo * ld, bytes, stream);
+  CK(cudaMemcpy2DAsync(out, sizeof(double) * p->n, data + (size_t)c_lo * ld,
                        sizeof(double) * ld, sizeof(double) * p->n, (size_t)(c_hi - c_lo), cudaMemcpyHostToDevice, stream));
   return ICIKT_OK;
 }
@@ -904,7 +919,7 @@ int64_t icikt_plan_num_pairs(const icikt_plan* p) { return p ? p->P : 0; }
 
 int icikt_plan_upload(icikt_plan* p, const double* data, int64_t ld) {
   if (!p || !data || ld < p->n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
-  return upload_columns(p, dense_source(data, ld), 0, p->C);
+  return upload_columns(p, dense_source(data, ld, p->C), 0, p->C);
 }
 
 int icikt_plan_set_device_matrix(icikt_plan* p, const double* d_data, int64_t ld) {
@@ -918,6 +933,17 @@ int icikt_plan_set_device_matrix(icikt_plan* p, const double* d_data, int64_t ld
   CK(cudaEventRecord(p->ev[0], p->stream));
   CK(cudaEventRecord(p->ev[1], p->stream));
   return ICIKT_OK;
+}
+
+// the CSC columns uploaded and not expanded yet, expanded into d_data_own on the plan's stream; returns the
+// launches or < 0 (the error is set)
+static int expand_columns(icikt_plan* p) {
+  if (p->expand_hi <= p->expand_lo) return 0;
+  const int l = launch_csc_expand(p->d_colptr, p->d_rowidx, p->d_values, p->n, p->expand_lo, p->expand_hi,
+                                  p->d_data_own + (size_t)p->expand_dst * p->n, p->stream);
+  if (l < 0) return launch_fail("CSC expansion kernel"), -1;
+  p->expand_lo = p->expand_hi = p->expand_dst = 0;
+  return l;
 }
 
 // K1 over columns [col_lo, col_hi); `finish`: the statistics of every column are in place afterwards
@@ -945,13 +971,8 @@ static int plan_columns_impl(icikt_plan* p, const double* global_na, int32_t n_g
   if (reset) CK(cudaMemsetAsync(p->tab.max_tied, 0, 4 * sizeof(int32_t), p->stream));
   CK(cudaEventRecord(e0 ? e0 : p->ev[2], p->stream));
   // columns uploaded as CSC become dense first (their copies precede this point on the stream)
-  int expand_launches = 0;
-  if (p->expand_hi > p->expand_lo) {
-    expand_launches = launch_csc_expand(p->d_colptr, p->d_rowidx, p->d_values, p->n, p->expand_lo, p->expand_hi,
-                                        p->d_data_own, p->stream);
-    if (expand_launches < 0) return launch_fail("CSC expansion kernel");
-    p->expand_lo = p->expand_hi = 0;
-  }
+  const int expand_launches = expand_columns(p);
+  if (expand_launches < 0) return ICIKT_ERR_CUDA;
   // the largest tier decides whether the global scratch may be needed at all
   const int64_t n_units = (int64_t)p->units.size();
   const bool inplace_ok = p->opts.perspective != ICIKT_PERSPECTIVE_COMPLETE;  // that mode has no in-place kernel
@@ -1016,7 +1037,7 @@ int icikt_plan_columns_finish(icikt_plan* p) {
 int icikt_plan_upload_columns(icikt_plan* p, const double* data, int64_t ld, int64_t col_lo, int64_t col_hi) {
   if (!p || !data || ld < p->n || col_lo < 0 || col_hi > p->C || col_lo > col_hi)
     return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
-  return upload_columns(p, dense_source(data, ld), col_lo, col_hi);
+  return upload_columns(p, dense_source(data, ld, p->C), col_lo, col_hi);
 }
 
 int icikt_plan_tables(icikt_plan* p, icikt_table* out, int32_t cap) {
@@ -1603,7 +1624,7 @@ int icikt_all_pairs(const double* data, int64_t n, int64_t C, int64_t ld, const 
                     int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue,
                     double* taumax, double* completeness, int32_t* status, int64_t* counts,
                     double* max_taumax, icikt_timings* timings) {
-  return one_shot(dense_source(data, ld), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw, pvalue,
+  return one_shot(dense_source(data, ld, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw, pvalue,
                   taumax, completeness, status, counts, max_taumax, timings);
 }
 
@@ -1613,7 +1634,7 @@ int icikt_all_pairs_csc(const int64_t* colptr, const int32_t* rowidx, const doub
                         double* max_taumax, icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return one_shot(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw,
+  return one_shot(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw,
                   pvalue, taumax, completeness, status, counts, max_taumax, timings);
 }
 
@@ -1642,7 +1663,7 @@ int icikt_matrices(const double* data, int64_t n, int64_t C, int64_t ld, const d
                    int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
                    double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
                    double* max_taumax, icikt_timings* timings) {
-  return matrices_impl(dense_source(data, ld), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max, diag_good,
+  return matrices_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max, diag_good,
                        n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
 }
 
@@ -1653,7 +1674,7 @@ int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const doubl
                        int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return matrices_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max,
+  return matrices_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max,
                        diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
 }
 
@@ -1664,11 +1685,13 @@ int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const doubl
 struct icikt_edges {
   std::vector<EdgeRow> rows;
   std::vector<double> cor;
+  int32_t j_offset = 0;  // a cross call's Cx: rows hold j as the matrix column of [X | Y], icikt_edges_copy gives Y's
 };
 
-// Pairs per window of the filtered calls, edges and top-k (ICIKT_EDGE_WINDOW, at most 2^30).  The default 2^26
+// Pairs per window of the filtered calls, edges, top-k and cross (ICIKT_EDGE_WINDOW, at most 2^30).  The default 2^26
 // keeps the window's buffers near 10 GB: the plan's pair buffers (68 B per pair) and the edge call's two
-// selected-row buffers (40 B each) or the top-k call's candidates (16 B).
+// selected-row buffers (40 B each), the top-k call's candidates (16 B) or the cross per-pair call's two result
+// buffers (36 B each).
 static int64_t edge_window() {
   const char* e = std::getenv("ICIKT_EDGE_WINDOW");
   const long long v = e ? std::atoll(e) : 0;
@@ -1698,20 +1721,33 @@ static int check_window_args(const ColumnSource& s, int64_t n, int64_t C, const 
   return ICIKT_OK;
 }
 
-static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                           const icikt_opts& o, const icikt_edge_filter* f, icikt_edges** out) {
+// the filter and the result pointer of the edge calls
+static int check_filter_args(const icikt_edge_filter* f, icikt_edges** out) {
   if (!out) return fail(ICIKT_ERR_BAD_ARG, "out is NULL");
   *out = nullptr;
   if (!f) return fail(ICIKT_ERR_BAD_ARG, "filter is NULL");
   if (f->max_edges < 0) return fail(ICIKT_ERR_BAD_ARG, "max_edges must be >= 0 (0: no limit)");
-  return check_window_args(s, n, C, global_na, n_global_na, o);
+  return ICIKT_OK;
+}
+
+static int check_edge_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                           const icikt_opts& o, const icikt_edge_filter* f, icikt_edges** out) {
+  const int rc = check_filter_args(f, out);
+  return rc == ICIKT_OK ? check_window_args(s, n, C, global_na, n_global_na, o) : rc;
+}
+
+// k and by of the top-k calls
+static int check_k_by(int32_t k, int32_t by) {
+  if (k < 1 || k > ICIKT_TOPK_MAX) return fail(ICIKT_ERR_BAD_ARG, "k must be in [1, ICIKT_TOPK_MAX]");
+  if (by != ICIKT_TOPK_ABS && by != ICIKT_TOPK_SIGNED)
+    return fail(ICIKT_ERR_BAD_ARG, "by must be ICIKT_TOPK_ABS or ICIKT_TOPK_SIGNED");
+  return ICIKT_OK;
 }
 
 static int check_topk_args(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
                            const icikt_opts& o, int32_t k, int32_t by, const int32_t* index) {
-  if (k < 1 || k > ICIKT_TOPK_MAX) return fail(ICIKT_ERR_BAD_ARG, "k must be in [1, ICIKT_TOPK_MAX]");
-  if (by != ICIKT_TOPK_ABS && by != ICIKT_TOPK_SIGNED)
-    return fail(ICIKT_ERR_BAD_ARG, "by must be ICIKT_TOPK_ABS or ICIKT_TOPK_SIGNED");
+  const int rc = check_k_by(k, by);
+  if (rc != ICIKT_OK) return rc;
   if (!index) return fail(ICIKT_ERR_BAD_ARG, "index is NULL");
   if (o.include_diag) return fail(ICIKT_ERR_BAD_ARG, "the top-k call ranks partners d != c: include_diag must be 0");
   return check_window_args(s, n, C, global_na, n_global_na, o);
@@ -1747,24 +1783,31 @@ static int ensure_edge_buffers(icikt_plan* p, int64_t W) {
   return ICIKT_OK;
 }
 
-// the top-k selection's buffers: candidates of a window of W pairs, and lists of k entries per column
-static int ensure_topk_buffers(icikt_plan* p, int64_t W, int k) {
+// the top-k selection's buffers: candidates of a window of W pairs, and lists of k entries for L columns (C, or the
+// requested sides of a cross call)
+static int ensure_topk_buffers(icikt_plan* p, int64_t W, int k, int64_t L) {
   const int rc = ensure_walk_buffers(p);
   if (rc != ICIKT_OK) return rc;
-  if (!p->d_tcol) {
-    ECK(dmalloc(&p->d_tcount, (size_t)p->C));
-    ECK(dmalloc(&p->d_tcand, 2 * (size_t)W));
-    ECK(dmalloc(&p->d_tcol, (size_t)p->C));
+  if (!p->d_tcand) ECK(dmalloc(&p->d_tcand, 2 * (size_t)W));
+  if (L > p->topk_cols) {
+    cudaFree(p->d_tcount);
+    cudaFree(p->d_tcol);
+    p->d_tcount = nullptr;
+    p->d_tcol = nullptr;
+    p->topk_cols = 0;
+    ECK(dmalloc(&p->d_tcount, (size_t)L));
+    ECK(dmalloc(&p->d_tcol, (size_t)L));
+    p->topk_cols = L;
   }
-  if (k > p->topk_cap) {
+  if (L * k > p->topk_entries) {
     cudaFree(p->d_tidx);
     cudaFree(p->d_tlist);
     p->d_tidx = nullptr;
     p->d_tlist = nullptr;
-    p->topk_cap = 0;
-    ECK(dmalloc(&p->d_tidx, (size_t)p->C * k));
-    ECK(dmalloc(&p->d_tlist, 4 * (size_t)p->C * k));
-    p->topk_cap = k;
+    p->topk_entries = 0;
+    ECK(dmalloc(&p->d_tidx, (size_t)(L * k)));
+    ECK(dmalloc(&p->d_tlist, 4 * (size_t)(L * k)));
+    p->topk_entries = L * k;
   }
   return ICIKT_OK;
 }
@@ -1812,34 +1855,61 @@ struct WalkTotals {
   unsigned long long bits = 0;
 };
 
-// upload and K1 of the single-device filtered calls, ahead of their window walk
-static int window_columns(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na) {
-  const int rc = upload_columns(p, s, 0, p->C);
-  return rc == ICIKT_OK ? plan_columns_impl(p, global_na, n_global_na, 0, p->C, true) : rc;
+// upload and K1 of the single-device filtered calls, ahead of their window walk.  A cross call passes Y as `y`: its
+// columns land behind X's, and K1 runs once over all columns of [X | Y].
+static int window_columns(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
+                          const ColumnSource* y = nullptr) {
+  int rc = upload_columns(p, s, 0, s.C);
+  int x_launches = 0;
+  if (rc == ICIKT_OK && y) {
+    // X's CSC arrays occupy the plan's CSC buffers, which Y's overwrite (and may reallocate): X is expanded first
+    x_launches = expand_columns(p);
+    if (x_launches < 0) return ICIKT_ERR_CUDA;
+    if (x_launches > 0 && y->csc()) CK(cudaStreamSynchronize(p->stream));
+    rc = copy_columns_in(p, *y, 0, y->C, p->stream, s.C);
+    if (rc != ICIKT_OK) return rc;
+    CK(cudaEventRecord(p->ev[1], p->stream));
+  }
+  if (rc == ICIKT_OK) rc = plan_columns_impl(p, global_na, n_global_na, 0, p->C, true);
+  p->tm.n_launches += x_launches;
+  return rc;
+}
+
+// The unit builders of the two pair orders the window walk knows, for pairs [lo, hi) with slots from lo.
+// combn order (all-pairs calls; the diagonal follows if include_diag):
+static auto combn_order(const icikt_plan* p) {
+  return [C = p->C, diag = p->opts.include_diag != 0](int64_t lo, int64_t hi, int64_t slots, std::vector<PairUnit>& U) {
+    int32_t row = 0, col = 0;
+    if (lo < tri_pairs(C)) icikt_pair_from_index(C, 0, lo, &row, &col);
+    range_units(C, diag, lo, hi, slots, U, row);
+  };
+}
+// cross order of Cx x Cy (icikt_cross.cuh):
+static auto cross_order(int64_t Cx, int64_t Cy) {
+  return [Cx, Cy](int64_t lo, int64_t hi, int64_t slots, std::vector<PairUnit>& U) { cross_units(Cx, Cy, lo, hi, slots, U); };
 }
 
 // The window walk of the filtered calls, on a plan whose pair buffers hold W pairs and whose columns are prepared
-// (K1 enqueued): pairs [first, last) of the pair order in windows of W.  Window w is enqueued (units, K2, K3,
+// (K1 enqueued): pairs [first, last) of a pair order in windows of W; order(lo, hi, slots, U) appends the units of
+// pairs [lo, hi) (combn_order or cross_order).  Window w is enqueued (units, K2, K3,
 // `select`, the readback of the maximum so far) before the host waits for window w - 1 and runs `collect` for it;
 // d_maxbits is not reset between windows, so K3's atomicMax leaves that maximum.  select(w, b, units, n_units,
 // n_slots) enqueues the selection of window w on p->stream (b: its buffer, 0 or 1); collect(w, b) runs once that
 // has completed.
-template <class Select, class Collect>
-static int walk_windows(icikt_plan* p, int64_t first, int64_t last, int64_t W, WalkTotals& tot, Select&& select,
-                        Collect&& collect) {
+template <class Order, class Select, class Collect>
+static int walk_windows(icikt_plan* p, const Order& order, int64_t first, int64_t last, int64_t W, WalkTotals& tot,
+                        Select&& select, Collect&& collect) {
   tot.launches = p->tm.n_launches;
   CK(cudaMemsetAsync(p->d_maxbits, 0, sizeof(unsigned long long), p->stream));
-  const int64_t nwin = (last - first + W - 1) / W, ptri = tri_pairs(p->C), slots = (int64_t)p->n_sm * 2;
+  const int64_t nwin = (last - first + W - 1) / W, slots = (int64_t)p->n_sm * 2;
   std::vector<PairUnit> U;
   int rc = ICIKT_OK;
 
   auto enqueue = [&](int64_t w) -> int {
     const int b = (int)(w & 1);
     const int64_t lo = first + w * W, hi = std::min(last, lo + W);
-    int32_t row = 0, col = 0;
-    if (lo < ptri) icikt_pair_from_index(p->C, 0, lo, &row, &col);
     U.clear();
-    range_units(p->C, p->opts.include_diag != 0, lo, hi, slots, U, row);
+    order(lo, hi, slots, U);
     int r = ensure_window_units(p, U.size());
     if (r != ICIKT_OK) return r;
     // the buffer was last read by window w - 2, whose selection the host has waited for
@@ -1914,8 +1984,9 @@ static int edge_limit_fail(const icikt_edge_filter& f, int64_t held, const std::
 // count; once the host has waited for a window, its rows are copied out on the copy stream and appended to `rows`,
 // and the rows held are re-trimmed against the new maximum (this walk's own: at most the final one, so the rows
 // stay a superset of the final edges).  The plan's edge buffers hold windows of W pairs.
-static int edge_walk(icikt_plan* p, const icikt_edge_filter& f, int64_t first, int64_t last, int64_t W,
-                     std::vector<EdgeRow>& rows, EdgeHeld& held, WalkTotals& tot, float& d2h_ms) {
+template <class Order>
+static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter& f, int64_t first, int64_t last,
+                     int64_t W, std::vector<EdgeRow>& rows, EdgeHeld& held, WalkTotals& tot, float& d2h_ms) {
   const double t = f.min_abs_cor;
   const bool scale = f.scale_max != 0;
   const bool retrim = scale && t == t;
@@ -1980,7 +2051,7 @@ static int edge_walk(icikt_plan* p, const icikt_edge_filter& f, int64_t first, i
     return ICIKT_OK;
   };
 
-  return walk_windows(p, first, last, W, tot, select, collect);
+  return walk_windows(p, order, first, last, W, tot, select, collect);
 }
 
 // The end of the filtered call, on one device or several: the rows held, in pair order, get the exact predicate with
@@ -2002,17 +2073,19 @@ static int edge_result(icikt_edges* res, const icikt_edge_filter& f, double M) {
   return ICIKT_OK;
 }
 
-// The filtered call on one device: upload, K1, the walk over the whole pair order, the final trim.
+// The filtered call on one device: upload, K1, the walk over the whole pair order, the final trim.  y: Y of a cross
+// call (the cross order), or null (combn order).
 static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
                         const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
-                        icikt_timings* timings) {
+                        icikt_timings* timings, const ColumnSource* y = nullptr) {
   int rc = ensure_edge_buffers(p, W);
-  if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na);
+  if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na, y);
   if (rc != ICIKT_OK) return rc;
   WalkTotals tot;
   float d2h_ms = 0.f;
   EdgeHeld held;
-  rc = edge_walk(p, f, 0, ptot, W, res->rows, held, tot, d2h_ms);
+  rc = y ? edge_walk(p, cross_order(s.C, y->C), f, 0, ptot, W, res->rows, held, tot, d2h_ms)
+         : edge_walk(p, combn_order(p), f, 0, ptot, W, res->rows, held, tot, d2h_ms);
   if (rc != ICIKT_OK) return rc;
   const double M = max_of_bits(tot.bits);
   rc = edge_result(res, f, M);
@@ -2031,11 +2104,14 @@ struct TopkOut {
   double *cor, *raw, *pvalue, *taumax, *completeness;
 };
 
-// The top-k call's walk over pairs [first, last): the lists start empty and every window's candidates are merged
-// into them on the device.  The plan's top-k buffers hold windows of W pairs and lists of k entries.
-static int topk_walk(icikt_plan* p, int k, int by, int64_t first, int64_t last, int64_t W, WalkTotals& tot) {
-  const int64_t C = p->C, ck = C * k;
-  CK(cudaMemsetAsync(p->d_tcol, 0, sizeof(TopkCol) * (size_t)C, p->stream));
+// The top-k call's walk over pairs [first, last) of `order`: the lists of columns [c_lo, c_hi) start empty and every
+// window's candidates are merged into them on the device.  The plan's top-k buffers hold windows of W pairs and
+// lists of k entries for those columns.
+template <class Order>
+static int topk_walk(icikt_plan* p, const Order& order, int64_t c_lo, int64_t c_hi, int k, int by, int64_t first,
+                     int64_t last, int64_t W, WalkTotals& tot) {
+  const int64_t ck = (c_hi - c_lo) * k;
+  CK(cudaMemsetAsync(p->d_tcol, 0, sizeof(TopkCol) * (size_t)(c_hi - c_lo), p->stream));
   auto select = [&](int64_t, int b, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
     TopkSelect ts;
     ts.units = units;
@@ -2046,7 +2122,8 @@ static int topk_walk(icikt_plan* p, int k, int by, int64_t first, int64_t last, 
     ts.taumax = p->d_tm;
     ts.completeness = p->d_comp;
     ts.status = p->d_status;
-    ts.C = C;
+    ts.c_lo = c_lo;
+    ts.c_hi = c_hi;
     ts.k = k;
     ts.by = by;
     ts.col_count = p->d_tcount;
@@ -2063,7 +2140,7 @@ static int topk_walk(icikt_plan* p, int k, int by, int64_t first, int64_t last, 
     tot.launches += l;
     return ICIKT_OK;
   };
-  return walk_windows(p, first, last, W, tot, select, [](int64_t, int) { return ICIKT_OK; });
+  return walk_windows(p, order, first, last, W, tot, select, [](int64_t, int) { return ICIKT_OK; });
 }
 
 // raw for cor when the caller wants cor but not raw
@@ -2102,12 +2179,12 @@ static void topk_fill_host(const TopkOut& out, int64_t C, int k, Held&& held, co
 static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na, int k,
                         int by, bool scale, int64_t ptot, int64_t W, const TopkOut& out, double* max_taumax,
                         icikt_timings* timings) {
-  int rc = ensure_topk_buffers(p, W, k);
+  int rc = ensure_topk_buffers(p, W, k, p->C);
   if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na);
   if (rc != ICIKT_OK) return rc;
   const int64_t C = p->C, ck = C * k;
   WalkTotals tot;
-  rc = topk_walk(p, k, by, 0, ptot, W, tot);
+  rc = topk_walk(p, combn_order(p), 0, C, k, by, 0, ptot, W, tot);
   if (rc != ICIKT_OK) return rc;
   // the lists, once
   std::vector<TopkCol> col;
@@ -2237,7 +2314,7 @@ extern "C" {
 int icikt_all_pairs_edges(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
                           int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
                           icikt_edges** out, double* max_taumax, icikt_timings* timings) {
-  return all_pairs_edges(dense_source(data, ld), n, C, global_na, n_global_na, opts, filter, out, max_taumax, timings);
+  return all_pairs_edges(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, filter, out, max_taumax, timings);
 }
 
 int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
@@ -2247,7 +2324,7 @@ int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, cons
   if (out) *out = nullptr;
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return all_pairs_edges(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, filter, out,
+  return all_pairs_edges(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, filter, out,
                          max_taumax, timings);
 }
 
@@ -2260,7 +2337,7 @@ int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, 
   for (size_t k = 0; k < m; ++k) {
     const EdgeRow& r = e->rows[k];
     if (i) i[k] = r.i;
-    if (j) j[k] = r.j;
+    if (j) j[k] = r.j - e->j_offset;
     if (raw) raw[k] = r.raw;
     if (pvalue) pvalue[k] = r.pvalue;
     if (taumax) taumax[k] = r.taumax;
@@ -2276,7 +2353,7 @@ int icikt_all_pairs_topk(const double* data, int64_t n, int64_t C, int64_t ld, c
                          int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
                          int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
                          double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
-  return all_pairs_topk(dense_source(data, ld), n, C, global_na, n_global_na, opts, k, by, scale_max,
+  return all_pairs_topk(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, k, by, scale_max,
                         TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
 }
 
@@ -2287,8 +2364,283 @@ int icikt_all_pairs_topk_csc(const int64_t* colptr, const int32_t* rowidx, const
                              double* max_taumax, icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return all_pairs_topk(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, k, by, scale_max,
+  return all_pairs_topk(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, k, by, scale_max,
                         TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
+}
+
+}  // extern "C"
+
+// ---- cross calls: every column of X against every column of Y (icikt_cross_pairs / _edges / _topk) ------------
+// The plan holds [X | Y] (Y from column Cx on) and K1 runs once over all Cx + Cy columns; the window walk covers the
+// cross order (icikt_cross.cuh), whose pair (i, j) is the plan's pair (i, Cx + j) staged with x column i.
+
+// One matrix of a cross call, checked on the host: exactly one form, C >= 1, ld >= n or a valid CSC matrix.
+static int cross_source(const icikt_input* in, const char* name, int64_t n, ColumnSource* out) {
+  const std::string m = std::string("matrix ") + name + ": ";
+  if (!in) return fail(ICIKT_ERR_BAD_ARG, m + "the input descriptor is NULL");
+  if ((in->data != nullptr) == (in->colptr != nullptr))
+    return fail(ICIKT_ERR_BAD_ARG, m + "set exactly one of data (dense) and colptr (CSC)");
+  if (in->C < 1) return fail(ICIKT_ERR_BAD_ARG, m + "C must be >= 1");
+  if (in->data) {
+    if (in->ld < n) return fail(ICIKT_ERR_BAD_ARG, m + "ld must be >= n");
+    *out = dense_source(in->data, in->ld, in->C);
+    return ICIKT_OK;
+  }
+  const int rc = check_csc(in->colptr, in->rowidx, in->values, n, in->C);
+  if (rc != ICIKT_OK) return fail(rc, m + g_err);
+  *out = csc_source(in->colptr, in->rowidx, in->values, in->C);
+  return ICIKT_OK;
+}
+
+// The argument checks all cross calls share, before any device is touched.  `ranged`: the call takes pair_lo /
+// pair_hi (within [0, Cx Cy]); the others refuse them.
+static int check_cross_args(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts& o, bool ranged, ColumnSource* sx, ColumnSource* sy) {
+  if (n < 1) return fail(ICIKT_ERR_BAD_ARG, "n must be >= 1");
+  int rc = cross_source(x, "x", n, sx);
+  if (rc == ICIKT_OK) rc = cross_source(y, "y", n, sy);
+  if (rc != ICIKT_OK) return rc;
+  if (sx->C + sy->C > 2147483647LL) return fail(ICIKT_ERR_BAD_ARG, "too many columns: Cx + Cy > INT32_MAX");
+  if (n > tiled_max_n()) return fail(ICIKT_ERR_TOO_LONG, "n exceeds icikt_max_n()");
+  if (n_global_na < 0 || (n_global_na > 0 && !global_na)) return fail(ICIKT_ERR_BAD_ARG, "bad global_na");
+  if (o.include_diag) return fail(ICIKT_ERR_BAD_ARG, "a cross call has no diagonal: include_diag must be 0");
+  if (o.perspective != ICIKT_PERSPECTIVE_GLOBAL && o.perspective != ICIKT_PERSPECTIVE_LOCAL)
+    return fail(ICIKT_ERR_BAD_ARG, "a cross call takes the global or the local perspective");
+  if (o.kernel != ICIKT_KERNEL_TILED) return fail(ICIKT_ERR_BAD_ARG, "a cross call needs the tiled kernel");
+  if (o.want_counts) return fail(ICIKT_ERR_BAD_ARG, "a cross call returns no counts (want_counts)");
+  const int64_t ptot = sx->C * sy->C;
+  if (ranged ? (o.pair_lo < 0 || o.pair_hi < 0 || o.pair_lo > ptot || o.pair_hi > ptot ||
+                (o.pair_hi != 0 && o.pair_lo > o.pair_hi) || (o.pair_hi == 0 && o.pair_lo != 0))
+             : (o.pair_lo != 0 || o.pair_hi != 0))
+    return fail(ICIKT_ERR_BAD_ARG, ranged ? "pair_lo/pair_hi out of [0, Cx * Cy]"
+                                          : "this cross call covers all pairs: pair_lo and pair_hi must be 0");
+  return ICIKT_OK;
+}
+
+// The cross call's plan (g_cached_edges, windows of W pairs of the Cx + Cy columns of [X | Y]); the caller holds
+// g_cache_mu.
+static int cross_plan(int64_t n, int64_t C, int64_t W, icikt_opts o, icikt_plan** out) {
+  o.pair_lo = o.pair_hi = 0;
+  return window_plan(g_cached_edges, n, C, W, o, out);
+}
+
+// icikt_cross_pairs on one device: per window, the results move off the plan's pair buffers into d_cres[b] on the
+// compute stream (the next window's K3 overwrites those buffers), and the host copies them from there into the
+// caller's arrays on the copy stream while the next window computes.
+static int cross_pair_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
+                              int32_t n_global_na, int64_t first, int64_t last, int64_t W, double* raw, double* pvalue,
+                              double* taumax, double* completeness, int32_t* status, double* max_taumax,
+                              icikt_timings* timings) {
+  int rc = ensure_walk_buffers(p);
+  if (rc != ICIKT_OK) return rc;
+  const size_t win = (size_t)p->P;  // the plan's pair buffers: W pairs and more
+  for (int b = 0; b < 2; ++b)
+    if (!p->d_cres[b] && cudaMalloc(reinterpret_cast<void**>(&p->d_cres[b]), win * (4 * sizeof(double) + sizeof(int32_t))) != cudaSuccess) {
+      cudaGetLastError();
+      return fail(ICIKT_ERR_ALLOC, "device allocation of the cross call's result windows failed");
+    }
+  rc = window_columns(p, sx, global_na, n_global_na, &sy);
+  if (rc != ICIKT_OK) return rc;
+  const double* d_field[4] = {p->d_tau, p->d_p, p->d_tm, p->d_comp};
+  double* host_field[4] = {raw, pvalue, taumax, completeness};
+  WalkTotals tot;
+  float d2h_ms = 0.f;
+  auto select = [&](int64_t, int b, const PairUnit*, int64_t, int64_t n_slots) -> int {
+    double* to = reinterpret_cast<double*>(p->d_cres[b]);
+    for (int f = 0; f < 4; ++f)
+      if (host_field[f])
+        CK(cudaMemcpyAsync(to + f * win, d_field[f], sizeof(double) * (size_t)n_slots, cudaMemcpyDeviceToDevice, p->stream));
+    if (status)
+      CK(cudaMemcpyAsync(to + 4 * win, p->d_status, sizeof(int32_t) * (size_t)n_slots, cudaMemcpyDeviceToDevice, p->stream));
+    return ICIKT_OK;
+  };
+  auto collect = [&](int64_t w, int b) -> int {
+    const int64_t off = w * W, cnt = std::min(W, last - first - off);
+    const double* from = reinterpret_cast<const double*>(p->d_cres[b]);
+    CK(cudaEventRecord(p->ev[6], p->copy_stream));
+    int r = ICIKT_OK;
+    for (int f = 0; f < 4 && r == ICIKT_OK; ++f)
+      if (host_field[f])
+        r = staged_copy_out(p, host_field[f] + off, from + f * win, sizeof(double) * (size_t)cnt, p->copy_stream);
+    if (r == ICIKT_OK && status)
+      r = staged_copy_out(p, status + off, from + 4 * win, sizeof(int32_t) * (size_t)cnt, p->copy_stream);
+    if (r != ICIKT_OK) return r;
+    CK(cudaEventRecord(p->ev[7], p->copy_stream));
+    CK(cudaEventSynchronize(p->ev[7]));
+    d2h_ms += ev_ms(p->ev[6], p->ev[7]);
+    return ICIKT_OK;
+  };
+  rc = walk_windows(p, cross_order(sx.C, sy.C), first, last, W, tot, select, collect);
+  if (rc == ICIKT_OK) rc = finish_walk(p, tot, d2h_ms, timings);
+  if (rc != ICIKT_OK) return rc;
+  if (max_taumax) *max_taumax = max_of_bits(tot.bits);
+  return ICIKT_OK;
+}
+
+static int cross_pairs(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                       int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
+                       double* completeness, int32_t* status, double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  ColumnSource sx, sy;
+  int rc = check_cross_args(x, y, n, global_na, n_global_na, o, true, &sx, &sy);
+  if (rc != ICIKT_OK) return rc;
+  if (!raw) return fail(ICIKT_ERR_BAD_ARG, "raw is NULL");
+  rc = select_device(o.device);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t first = o.pair_lo, last = (o.pair_hi == 0) ? sx.C * sy.C : o.pair_hi;
+  if (last == first) {  // an empty slice: nothing to compute
+    if (max_taumax) *max_taumax = std::nan("");
+    if (timings) std::memset(timings, 0, sizeof(*timings));
+    return ICIKT_OK;
+  }
+  const int64_t W = std::min(edge_window(), last - first);
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  icikt_plan* p = nullptr;
+  rc = cross_plan(n, sx.C + sy.C, W, o, &p);
+  if (rc == ICIKT_OK)
+    rc = cross_pair_windows(p, sx, sy, global_na, n_global_na, first, last, W, raw, pvalue, taumax, completeness, status,
+                            max_taumax, timings);
+  if (rc != ICIKT_OK) drop_window_plan(g_cached_edges);
+  return rc;
+}
+
+static int cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                       int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
+                       double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  ColumnSource sx, sy;
+  int rc = check_filter_args(filter, out);
+  if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
+  if (rc != ICIKT_OK) return rc;
+  rc = select_device(o.device);
+  if (rc != ICIKT_OK) return rc;
+  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
+  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
+  res->j_offset = (int32_t)sx.C;
+  const int64_t ptot = sx.C * sy.C, W = std::min(edge_window(), ptot);
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  icikt_plan* p = nullptr;
+  rc = cross_plan(n, sx.C + sy.C, W, o, &p);
+  if (rc == ICIKT_OK) rc = edge_windows(p, sx, global_na, n_global_na, *filter, ptot, W, res.get(), max_taumax, timings, &sy);
+  if (rc != ICIKT_OK) {
+    drop_window_plan(g_cached_edges);
+    return rc;
+  }
+  *out = res.release();
+  return ICIKT_OK;
+}
+
+// icikt_cross_topk on one device: lists for the columns of the requested sides only, [c_lo, c_hi) of [X | Y] (X's
+// columns come first, so any choice of sides is one range); after the last window each side's rows of the lists go
+// to its caller arrays, and an x-side partner (a column Cx + j of the plan) becomes Y's index j.
+static int cross_topk_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
+                              int32_t n_global_na, int k, int by, bool scale, int64_t W, const icikt_topk_lists* x_side,
+                              const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings) {
+  const int64_t Cx = sx.C, Cy = sy.C;
+  const int64_t c_lo = x_side ? 0 : Cx, c_hi = y_side ? Cx + Cy : Cx, L = c_hi - c_lo;
+  int rc = ensure_topk_buffers(p, W, k, L);
+  if (rc == ICIKT_OK) rc = window_columns(p, sx, global_na, n_global_na, &sy);
+  if (rc != ICIKT_OK) return rc;
+  WalkTotals tot;
+  rc = topk_walk(p, cross_order(Cx, Cy), c_lo, c_hi, k, by, 0, Cx * Cy, W, tot);
+  if (rc != ICIKT_OK) return rc;
+  struct Side {
+    TopkOut out;
+    int64_t row0, cols;  // its first list row and its columns
+    int32_t shift;       // subtracted from its partners
+    std::vector<double> raw_own;
+    double* raw = nullptr;
+  };
+  std::vector<Side> sides;
+  if (x_side) sides.push_back(Side{TopkOut{x_side->index, x_side->n_neighbors, x_side->cor, x_side->raw, x_side->pvalue,
+                                           x_side->taumax, x_side->completeness}, 0, Cx, (int32_t)Cx, {}, nullptr});
+  if (y_side) sides.push_back(Side{TopkOut{y_side->index, y_side->n_neighbors, y_side->cor, y_side->raw, y_side->pvalue,
+                                           y_side->taumax, y_side->completeness}, Cx - c_lo, Cy, 0, {}, nullptr});
+  std::vector<TopkCol> col;
+  try {
+    col.resize((size_t)L);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
+  }
+  CK(cudaEventRecord(p->ev[6], p->stream));
+  rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)L, p->stream);
+  const int64_t lk = L * k;
+  for (Side& sd : sides) {
+    const int64_t ck = sd.cols * k, at = sd.row0 * k;
+    if (rc == ICIKT_OK) rc = topk_raw_buffer(sd.out, ck, sd.raw_own, &sd.raw);
+    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index, p->d_tidx + at, sizeof(int32_t) * (size_t)ck, p->stream);
+    double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
+    for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
+      if (host_field[f])
+        rc = staged_copy_out(p, host_field[f], p->d_tlist + f * lk + at, sizeof(double) * (size_t)ck, p->stream);
+  }
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[7], p->stream));
+  CK(cudaEventSynchronize(p->ev[7]));
+  const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
+  const double M = max_of_bits(tot.bits);
+  for (Side& sd : sides) {
+    auto held = [&](int64_t c) { return (int64_t)col[(size_t)(sd.row0 + c)].n; };
+    if (sd.shift)
+      for (int64_t c = 0; c < sd.cols; ++c)
+        for (int64_t r = 0, h = held(c); r < h; ++r) sd.out.index[c * k + r] -= sd.shift;
+    topk_fill_host(sd.out, sd.cols, k, held, sd.raw, scale, M);
+  }
+  rc = finish_walk(p, tot, d2h_ms, timings);
+  if (rc != ICIKT_OK) return rc;
+  if (max_taumax) *max_taumax = M;
+  return ICIKT_OK;
+}
+
+static int cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                      const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
+                      icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  int rc = check_k_by(k, by);
+  if (rc != ICIKT_OK) return rc;
+  if (!x_side && !y_side) return fail(ICIKT_ERR_BAD_ARG, "x_side and y_side are both NULL");
+  if ((x_side && !x_side->index) || (y_side && !y_side->index))
+    return fail(ICIKT_ERR_BAD_ARG, x_side && !x_side->index ? "x_side->index is NULL" : "y_side->index is NULL");
+  ColumnSource sx, sy;
+  rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
+  if (rc != ICIKT_OK) return rc;
+  rc = select_device(o.device);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t W = std::min(edge_window(), sx.C * sy.C);
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  icikt_plan* p = nullptr;
+  rc = cross_plan(n, sx.C + sy.C, W, o, &p);
+  if (rc == ICIKT_OK)
+    rc = cross_topk_windows(p, sx, sy, global_na, n_global_na, k, by, scale_max != 0, W, x_side, y_side, max_taumax,
+                            timings);
+  if (rc != ICIKT_OK) drop_window_plan(g_cached_edges);
+  return rc;
+}
+
+extern "C" {
+
+int icikt_cross_pairs(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
+                      double* completeness, int32_t* status, double* max_taumax, icikt_timings* timings) {
+  return cross_pairs(x, y, n, global_na, n_global_na, opts, raw, pvalue, taumax, completeness, status, max_taumax,
+                     timings);
+}
+
+int icikt_cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
+                      double* max_taumax, icikt_timings* timings) {
+  return cross_edges(x, y, n, global_na, n_global_na, opts, filter, out, max_taumax, timings);
+}
+
+int icikt_cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                     int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                     const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
+                     icikt_timings* timings) {
+  return cross_topk(x, y, n, global_na, n_global_na, opts, k, by, scale_max, x_side, y_side, max_taumax, timings);
 }
 
 }  // extern "C"
@@ -2384,7 +2736,7 @@ extern "C" {
 int icikt_pairwise_completeness(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
                                 int32_t n_global_na, int32_t device, const int32_t* pi, const int32_t* pj,
                                 int64_t P, int32_t* missing, double* completeness, double* matrix) {
-  return pairwise_completeness_impl(dense_source(data, ld), n, C, global_na, n_global_na, device, pi, pj, P, missing,
+  return pairwise_completeness_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, device, pi, pj, P, missing,
                                     completeness, matrix);
 }
 
@@ -2394,7 +2746,7 @@ int icikt_pairwise_completeness_csc(const int64_t* colptr, const int32_t* rowidx
                                     double* completeness, double* matrix) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return pairwise_completeness_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, device, pi, pj,
+  return pairwise_completeness_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, device, pi, pj,
                                     P, missing, completeness, matrix);
 }
 
@@ -2787,7 +3139,7 @@ int edges_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* 
           WalkTotals tot;
           float d2h_ms = 0.f;
           w.rc = ensure_edge_buffers(p, p->P);
-          if (w.rc == ICIKT_OK) w.rc = edge_walk(p, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
+          if (w.rc == ICIKT_OK) w.rc = edge_walk(p, combn_order(p), f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
           if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
           bits[(size_t)k] = tot.bits;
         }
@@ -2911,8 +3263,8 @@ int topk_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* g
         w.rc = window_multi_worker(J, k, &p);
         if (w.rc == ICIKT_OK) {
           WalkTotals tot;
-          w.rc = ensure_topk_buffers(p, p->P, K);
-          if (w.rc == ICIKT_OK) w.rc = topk_walk(p, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
+          w.rc = ensure_topk_buffers(p, p->P, K, J.C);
+          if (w.rc == ICIKT_OK) w.rc = topk_walk(p, combn_order(p), 0, J.C, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
           if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, 0.f, &w.tm);
           bits[(size_t)k] = tot.bits;
         }
@@ -2949,7 +3301,7 @@ int icikt_all_pairs_multi(const double* data, int64_t n, int64_t C, int64_t ld, 
                           int32_t n_devices, double* raw, double* pvalue, double* taumax,
                           double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
                           icikt_timings* timings) {
-  return all_pairs_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, raw,
+  return all_pairs_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, raw,
                               pvalue, taumax, completeness, status, counts, max_taumax, timings);
 }
 
@@ -2960,7 +3312,7 @@ int icikt_all_pairs_multi_csc(const int64_t* colptr, const int32_t* rowidx, cons
                               icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return all_pairs_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices,
+  return all_pairs_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices,
                               n_devices, raw, pvalue, taumax, completeness, status, counts, max_taumax, timings);
 }
 
@@ -2969,7 +3321,7 @@ int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, c
                          int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
                          double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
                          double* max_taumax, icikt_timings* timings) {
-  return matrices_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, scale_max,
+  return matrices_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, scale_max,
                              diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax,
                              timings);
 }
@@ -2982,7 +3334,7 @@ int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const
                              icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return matrices_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices,
+  return matrices_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices,
                              n_devices, scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness,
                              status_counts, max_taumax, timings);
 }
@@ -2991,7 +3343,7 @@ int icikt_all_pairs_edges_multi(const double* data, int64_t n, int64_t C, int64_
                                 int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
                                 const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
                                 icikt_timings* timings) {
-  return edges_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, filter, out,
+  return edges_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, filter, out,
                           max_taumax, timings);
 }
 
@@ -3002,7 +3354,7 @@ int icikt_all_pairs_edges_multi_csc(const int64_t* colptr, const int32_t* rowidx
   if (out) *out = nullptr;
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return edges_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices, n_devices,
+  return edges_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices, n_devices,
                           filter, out, max_taumax, timings);
 }
 
@@ -3011,7 +3363,7 @@ int icikt_all_pairs_topk_multi(const double* data, int64_t n, int64_t C, int64_t
                                int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
                                double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
                                double* max_taumax, icikt_timings* timings) {
-  return topk_multi_impl(dense_source(data, ld), n, C, global_na, n_global_na, opts, devices, n_devices, k, by,
+  return topk_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, k, by,
                          scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax,
                          timings);
 }
@@ -3023,7 +3375,7 @@ int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx,
                                    double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return topk_multi_impl(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, opts, devices, n_devices, k,
+  return topk_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices, n_devices, k,
                          by, scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness},
                          max_taumax, timings);
 }
@@ -3034,7 +3386,7 @@ int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const 
                     double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
                     icikt_timings* timings) {
   if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
-  return one_shot(dense_source(data, ld), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue, taumax,
+  return one_shot(dense_source(data, ld, C), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue, taumax,
                   completeness, status, counts, max_taumax, timings);
 }
 
@@ -3045,7 +3397,7 @@ int icikt_pair_list_csc(const int64_t* colptr, const int32_t* rowidx, const doub
   if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return one_shot(csc_source(colptr, rowidx, values), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue,
+  return one_shot(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue,
                   taumax, completeness, status, counts, max_taumax, timings);
 }
 

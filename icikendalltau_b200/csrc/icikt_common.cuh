@@ -49,6 +49,16 @@ constexpr int kDirectBudget = 24;
 constexpr int kLargeStride = 1024;  // u16 per column in the large-group table: (start, size) x 512
 constexpr unsigned kLargeFlag = 0x8000u;
 
+// A unit of pair work: column `col` is staged in shared memory and correlated with
+// `count` other columns; results go to slots [slot0, slot0+count).
+struct PairUnit {
+  int64_t slot0;
+  int32_t col;    // staged column
+  int32_t j0;     // other column of the first pair; the k-th pair uses j0 + k (j_explicit == 0)
+  int32_t count;
+  int32_t j_explicit;  // 1: other columns are pj_list[slot0 + k]
+};
+
 struct PairOut {
   double tau, pvalue, taumax, completeness;
   int64_t xtie, ytie, tot, n_entry, ntie;

@@ -49,16 +49,6 @@ struct ColumnTables {
   int32_t* max_tied = nullptr;    // [4] over the columns: [0] any large tie group, [1] max large groups, [2] max distinct values
 };
 
-// A unit of pair work: column `col` is staged in shared memory and correlated with
-// `count` other columns; results go to slots [slot0, slot0+count).
-struct PairUnit {
-  int64_t slot0;
-  int32_t col;    // staged column
-  int32_t j0;     // other column of the first pair; the k-th pair uses j0 + k (j_explicit == 0)
-  int32_t count;
-  int32_t j_explicit;  // 1: other columns are pj_list[slot0 + k]
-};
-
 struct PairRaw {  // what K2 hands to K3
   int64_t dis, ntie, b, g00;
 };
@@ -228,6 +218,8 @@ int launch_edge_select(const EdgeSelect& s, cudaStream_t stream);
 // every valid slot (column i gets partner j, column j gets i) against the column's k-th entry, one CTA scans the
 // column counts into bucket offsets, a scatter pass fills the buckets, and one CTA per column merges its bucket
 // into the column's sorted list (order of icikt_topk.cuh), gathering the new entries' fields from the window.
+// Lists are kept for columns [c_lo, c_hi) only (all columns, or one side of a cross call): a candidate for a column
+// outside that range is skipped, and every per-column array is indexed by c - c_lo.
 constexpr int kTopkMax = 1024;  // ICIKT_TOPK_MAX
 struct TopkCol {
   unsigned long long key;  // the k-th entry's key and partner, once n == k
@@ -240,14 +232,14 @@ struct TopkSelect {
   int64_t n_slots;        // pairs in the window
   const double *tau, *pvalue, *taumax, *completeness;
   const int32_t* status;
-  int64_t C;
+  int64_t c_lo, c_hi;     // the columns that keep lists; L = c_hi - c_lo below
   int k, by;
-  uint32_t* col_count;    // device [C]: candidates per column, then the end of every column's bucket
+  uint32_t* col_count;    // device [L]: candidates per column, then the end of every column's bucket
   unsigned long long* total;  // device, candidates in the window
   uint2* cand;            // device [2 n_slots]: (window slot, partner)
-  TopkCol* col;           // device [C], zero before the first window
-  int32_t* idx;           // device [C k]: the sorted lists
-  double *raw, *pv, *tm, *comp;  // device [C k]
+  TopkCol* col;           // device [L], zero before the first window
+  int32_t* idx;           // device [L k]: the sorted lists
+  double *raw, *pv, *tm, *comp;  // device [L k]
 };
 int launch_topk_select(const TopkSelect& s, cudaStream_t stream);
 

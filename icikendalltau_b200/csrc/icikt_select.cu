@@ -159,7 +159,8 @@ __global__ void __launch_bounds__(kSelThreads) edge_scatter_kernel(const EdgeSel
 
 // Top-k: the count pass (kScatter false) and the scatter pass (true) of one tile of kEdgeTile slots.  Both make
 // the same decisions, against the thresholds the previous window's merge left.  A unit's pairs share column i,
-// so its candidates for i are counted with one atomic per warp and column.
+// so its candidates for i are counted with one atomic per warp and column.  Columns outside [c_lo, c_hi) keep no
+// list and take no candidate; ri, rj are the list rows of i and j.
 __device__ __forceinline__ bool topk_takes(const TopkCol& t, int k, unsigned long long key, int32_t partner) {
   return t.n < k || topk_before(key, partner, t.key, t.idx);
 }
@@ -178,34 +179,37 @@ __global__ void __launch_bounds__(kSelThreads) topk_bucket_kernel(const TopkSele
   const long long ua = unit_range[0], ub = unit_range[1] + 1;
   for (int r = 0; r < kSelRounds; ++r) {
     const long long slot = tile * kEdgeTile + r * kSelThreads + threadIdx.x;
-    int32_t i = -1, j = -1;
+    int32_t i = -1, j = -1, ri = -1, rj = -1;
     bool take_i = false, take_j = false;
     if (slot < s.n_slots && s.status[slot] == 0) {
       const PairUnit u = s.units[unit_of(s.units, ua, ub, slot)];
       i = u.col;
       j = u.j0 + (int32_t)(slot - u.slot0);
+      ri = i - (int32_t)s.c_lo;
+      rj = j - (int32_t)s.c_lo;
+      const uint32_t L = (uint32_t)(s.c_hi - s.c_lo);
       const unsigned long long key = topk_key(s.tau[slot], s.by);
-      take_i = topk_takes(s.col[i], s.k, key, j);
-      take_j = topk_takes(s.col[j], s.k, key, i);
+      take_i = (uint32_t)ri < L && topk_takes(s.col[ri], s.k, key, j);
+      take_j = (uint32_t)rj < L && topk_takes(s.col[rj], s.k, key, i);
     }
     const unsigned peers = __match_any_sync(FULL, take_i ? i : -1);
     if (take_i) {
       const int leader = __ffs(peers) - 1;
       unsigned at = 0;
-      if (lane == leader) at = atomicAdd(&s.col_count[i], (unsigned)__popc(peers));
+      if (lane == leader) at = atomicAdd(&s.col_count[ri], (unsigned)__popc(peers));
       if (kScatter) {
         at = __shfl_sync(peers, at, leader) + __popc(peers & ((1u << lane) - 1u));
         s.cand[at] = make_uint2((unsigned)slot, (unsigned)j);
       }
     }
     if (take_j) {
-      const unsigned at = atomicAdd(&s.col_count[j], 1u);
+      const unsigned at = atomicAdd(&s.col_count[rj], 1u);
       if (kScatter) s.cand[at] = make_uint2((unsigned)slot, (unsigned)i);
     }
   }
 }
 
-// One CTA per column: its bucket is taken in chunks that fill a shared array behind the list; candidates that
+// One CTA per column that keeps a list (c below is its list row): its bucket is taken in chunks that fill a shared array behind the list; candidates that
 // cannot beat the list's k-th entry are dropped, the rest are sorted with the list (bitonic) and the first k
 // kept.  Then every thread gathers one entry's fields, from the list or from the window, before any is written.
 constexpr int kMergeThreads = kTopkMax;
@@ -387,14 +391,15 @@ int launch_topk_device_merge(const TopkDeviceMerge& m, cudaStream_t stream) {
 int launch_topk_select(const TopkSelect& s, cudaStream_t stream) {
   if (s.n_slots <= 0) return launch_status(0);
   const long long tiles = (s.n_slots + kEdgeTile - 1) / kEdgeTile;
-  if (tiles > 0x7fffffffLL || s.C > 0x7fffffffLL || 2 * s.n_slots > 0xffffffffLL)
+  const long long L = s.c_hi - s.c_lo;
+  if (tiles > 0x7fffffffLL || s.c_lo < 0 || L < 1 || s.c_hi > 0x7fffffffLL || 2 * s.n_slots > 0xffffffffLL)
     return launch_refused("top-k selection: window too large");
-  if (cudaMemsetAsync(s.col_count, 0, sizeof(uint32_t) * (size_t)s.C, stream) != cudaSuccess)
+  if (cudaMemsetAsync(s.col_count, 0, sizeof(uint32_t) * (size_t)L, stream) != cudaSuccess)
     return launch_refused("top-k selection: clearing the column counts");
   topk_bucket_kernel<false><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
-  edge_scan_kernel<<<1, 1024, 0, stream>>>(s.col_count, s.C, s.total);
+  edge_scan_kernel<<<1, 1024, 0, stream>>>(s.col_count, L, s.total);
   topk_bucket_kernel<true><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
-  topk_merge_kernel<<<(unsigned)s.C, kMergeThreads, 0, stream>>>(s);
+  topk_merge_kernel<<<(unsigned)L, kMergeThreads, 0, stream>>>(s);
   return launch_status(4);
 }
 

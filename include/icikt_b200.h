@@ -269,8 +269,9 @@ int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, cons
                               icikt_timings* timings);
 /* number of rows (0 for NULL) */
 int64_t icikt_edges_count(const icikt_edges* e);
-/* the rows into caller arrays of icikt_edges_count(e) entries; any pointer may be NULL.  i < j, or i == j for
- * the diagonal pairs; cor as defined above */
+/* the rows into caller arrays of icikt_edges_count(e) entries; any pointer may be NULL; cor as defined above.
+ * All-pairs result: i < j, or i == j for the diagonal pairs.  Cross result (icikt_cross_edges): i in [0, Cx) is
+ * X's column and j in [0, Cy) is Y's own column index. */
 int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, double* raw, double* pvalue,
                      double* taumax, double* completeness);
 void icikt_edges_free(icikt_edges* e);
@@ -352,6 +353,67 @@ int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx,
                                    const int32_t* devices, int32_t n_devices, int32_t k, int32_t by, int32_t scale_max,
                                    int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
                                    double* taumax, double* completeness, double* max_taumax, icikt_timings* timings);
+
+/* ---- cross calls: every column of a matrix X (n x Cx) against every column of a matrix Y (n x Cy) with the same n
+ * rows -- query samples against a reference panel, two batches, two feature sets measured on the same samples.
+ *
+ *   - Pair order: x-major, pair p = i * Cy + j is (x column i, y column j), so a per-pair array of the whole order is
+ *     the Cx x Cy matrix in row-major order.
+ *   - Exactness: X's column is the reference's `x` (first column).  Every field is bit for bit what icikt_pair_list
+ *     returns on the dense [X | Y] (ld = n) with pi = i and pj = Cx + j, and max_taumax is the maximum over the
+ *     computed pairs.  The per-column statistics of K1 depend on the column alone, so preprocessing [X | Y] gives
+ *     every column the tables it gets in that call.
+ *   - Input: each matrix is an icikt_input, dense or CSC (see the sparse calls above; CSC arrays are checked before
+ *     any device work, and a message names the matrix, x or y, and the column).
+ *   - Options: perspective global or local, alternative, continuity, na_inf, device, and (icikt_cross_pairs only)
+ *     pair_lo / pair_hi.  Refused with ICIKT_ERR_BAD_ARG before any device is touched: x or y NULL, a descriptor
+ *     with both forms or neither, C < 1, n < 1, ld < n, Cx + Cy > INT32_MAX, bad CSC, include_diag,
+ *     ICIKT_PERSPECTIVE_COMPLETE, ICIKT_KERNEL_NAIVE, want_counts, pair_lo / pair_hi outside [0, Cx * Cy] (non-zero
+ *     on the edges and top-k calls), and whatever icikt_all_pairs_edges / icikt_all_pairs_topk refuse of their own
+ *     arguments.  A well-formed call without a device returns ICIKT_ERR_NO_DEVICE.
+ *   - Device memory does not depend on the number of pairs: all three calls walk the cross order in windows of
+ *     ICIKT_EDGE_WINDOW pairs, as the filtered all-pairs calls do.  timings as there. */
+typedef struct icikt_input {
+  int64_t C;                 /* columns                                                   */
+  const double* data;        /* dense column-major, ld >= n; NULL for CSC                 */
+  int64_t ld;
+  const int64_t* colptr;     /* CSC as in the *_csc calls (C + 1 entries); NULL for dense */
+  const int32_t* rowidx;
+  const double* values;
+} icikt_input;
+
+/* Per-pair results of pairs [pair_lo, pair_hi) of the cross order (0, 0: all Cx * Cy), straight into caller arrays
+ * indexed from 0 = pair_lo.  pvalue / taumax / completeness / status / max_taumax / timings may be NULL, raw may not.
+ * Each window's results are copied to the caller while the next window is computed. */
+int icikt_cross_pairs(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
+                      double* completeness, int32_t* status, double* max_taumax, icikt_timings* timings);
+
+/* The filtered call (icikt_all_pairs_edges) on the cross order: the same filter, predicate, prefilter, final trim
+ * with M and max_edges.  Rows are in cross order; icikt_edges_copy gives i as X's and j as Y's column index. */
+int icikt_cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
+                      double* max_taumax, icikt_timings* timings);
+
+/* Each column's k best partners in the OTHER matrix, in the order of icikt_all_pairs_topk (|raw| or raw descending,
+ * then partner ascending; degenerate pairs are never candidates).  x_side receives Cx x k lists whose partners are Y
+ * indices, y_side Cy x k lists whose partners are X indices; entry r of column c at c * k + r, padding index -1 and a
+ * quiet NaN, k > the other side's width only pads.  Either side may be NULL, not both; a given side needs index, its
+ * other pointers may be NULL.  Lists are held on the device for the requested sides only: 36 B x k x their columns. */
+typedef struct icikt_topk_lists {
+  int32_t* index;        /* [C k] partner, -1 where unused      */
+  int32_t* n_neighbors;  /* [C] entries kept                    */
+  double* cor;           /* [C k] each, NaN where unused        */
+  double* raw;
+  double* pvalue;
+  double* taumax;
+  double* completeness;
+} icikt_topk_lists;
+
+int icikt_cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                     int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                     const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
+                     icikt_timings* timings);
 
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
