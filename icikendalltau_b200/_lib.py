@@ -41,6 +41,7 @@ EXPORTS = [
     "icikt_edges_free", "icikt_all_pairs_topk", "icikt_all_pairs_topk_csc",
     "icikt_all_pairs_edges_multi", "icikt_all_pairs_edges_multi_csc", "icikt_all_pairs_topk_multi",
     "icikt_all_pairs_topk_multi_csc", "icikt_cross_pairs", "icikt_cross_edges", "icikt_cross_topk",
+    "icikt_cross_pairs_multi", "icikt_cross_edges_multi", "icikt_cross_topk_multi",
 ]
 NSTATUS = 10
 
@@ -208,6 +209,11 @@ def load():
     L.icikt_cross_topk.argtypes = cross + [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(TopkLists),
                                            ctypes.POINTER(TopkLists), _dp, ctypes.POINTER(Timings)]
     L.icikt_cross_topk.restype = ctypes.c_int
+    for name in ("icikt_cross_pairs", "icikt_cross_edges", "icikt_cross_topk"):  # (devices, n_devices) after opts
+        a = getattr(L, name).argtypes
+        f = getattr(L, name + "_multi")
+        f.argtypes = a[:6] + [_ip, ctypes.c_int32] + a[6:]
+        f.restype = ctypes.c_int
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -479,13 +485,16 @@ def _cross_inputs(x, y):
     return ins[0], ins[1], nx, cx, cy, keep
 
 
-def run_cross(x, y, global_na=(), **opt_kw):
+def run_cross(x, y, global_na=(), devices=None, **opt_kw):
     """icikt_cross_pairs: every column of x against every column of y (same rows), pair p = i * Cy + j in x-major
     order; pair_lo / pair_hi select a slice (0, 0: all).  Every field is bit for bit run_pairs(hstack([x, y]),
-    pi=i, pj=Cx + j)'s.  x and y may each be a NumPy array or a scipy.sparse matrix.  Returns a dict of NumPy arrays
-    in pair order: raw, pvalue, taumax, completeness, status, plus max_taumax and timings."""
+    pi=i, pj=Cx + j)'s.  x and y may each be a NumPy array or a scipy.sparse matrix.  devices: list of CUDA
+    ordinals -> icikt_cross_pairs_multi: every device computes a contiguous slice of the pairs; the result is bit for
+    bit the single-device one.  Returns a dict of NumPy arrays in pair order: raw, pvalue, taumax, completeness,
+    status, plus max_taumax and timings."""
     L = load()
     xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    msfx, dargs, dev = _devices_args(devices)
     o = make_opts(**opt_kw)
     P = cx * cy if (o.pair_lo == 0 and o.pair_hi == 0) else max(o.pair_hi - o.pair_lo, 0)
     buf = np.empty(4 * P + (P + 1) // 2, dtype=np.float64)
@@ -495,25 +504,30 @@ def run_cross(x, y, global_na=(), **opt_kw):
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(L.icikt_cross_pairs(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o), a, a + 8 * P,
-                              a + 16 * P, a + 24 * P, a + 32 * P, ctypes.byref(mx), ctypes.byref(t)))
+    check(getattr(L, "icikt_cross_pairs" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
+                                                 *dargs, a, a + 8 * P, a + 16 * P, a + 24 * P, a + 32 * P,
+                                                 ctypes.byref(mx), ctypes.byref(t)))
     return dict(raw=raw, pvalue=pv, taumax=tm, completeness=comp, status=status, max_taumax=mx.value,
                 timings=t.as_dict())
 
 
-def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, **opt_kw):
+def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, devices=None,
+                    **opt_kw):
     """icikt_cross_edges: the pairs of x's columns with y's columns that pass the filter of run_edges, in cross
-    order, filtered on the device.  Returns the dict of run_edges; i indexes x's columns, j y's."""
+    order, filtered on the device.  devices: list of CUDA ordinals -> icikt_cross_edges_multi, bit for bit the
+    single-device result.  Returns the dict of run_edges; i indexes x's columns, j y's."""
     L = load()
     xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    msfx, dargs, dev = _devices_args(devices)
     o = make_opts(**opt_kw)
     f = EdgeFilter(_bound(min_abs_cor), _bound(max_pvalue), int(bool(scale_max)), 0, int(max_edges))
     h = ctypes.c_void_p()
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(L.icikt_cross_edges(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o), ctypes.byref(f),
-                              ctypes.byref(h), ctypes.byref(mx), ctypes.byref(t)))
+    check(getattr(L, "icikt_cross_edges" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
+                                                 *dargs, ctypes.byref(f), ctypes.byref(h), ctypes.byref(mx),
+                                                 ctypes.byref(t)))
     try:
         m = int(L.icikt_edges_count(h))
         out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
@@ -528,17 +542,20 @@ def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale
 CROSS_SIDES = {"x": (True, False), "y": (False, True), "both": (True, True)}
 
 
-def run_cross_topk(x, y, global_na=(), k=10, by="abs", scale_max=True, side="both", **opt_kw):
+def run_cross_topk(x, y, global_na=(), k=10, by="abs", scale_max=True, side="both", devices=None, **opt_kw):
     """icikt_cross_topk: each column's k best partners in the other matrix, in the order of run_topk.  side "x": the
-    lists of x's columns (partners are y indices), "y": of y's columns (partners are x indices), "both".  Returns a
-    dict with x_side and/or y_side (each the per-column arrays of run_topk: index, n_neighbors, cor, raw, pvalue,
-    taumax, completeness), max_taumax and timings."""
+    lists of x's columns (partners are y indices), "y": of y's columns (partners are x indices), "both".  devices:
+    list of CUDA ordinals -> icikt_cross_topk_multi: every device walks a contiguous slice of the pairs and the
+    devices merge their lists, bit for bit the single-device result.  Returns a dict with x_side and/or y_side (each
+    the per-column arrays of run_topk: index, n_neighbors, cor, raw, pvalue, taumax, completeness), max_taumax and
+    timings."""
     if by not in TOPK_BY:
         raise ValueError(f"by must be one of {sorted(TOPK_BY)}")
     if side not in CROSS_SIDES:
         raise ValueError(f"side must be one of {sorted(CROSS_SIDES)}")
     L = load()
     xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    msfx, dargs, dev = _devices_args(devices)
     o = make_opts(**opt_kw)
     k = int(k)
     kk = k if 1 <= k <= TOPK_MAX else 0  # a k the library refuses gets no arrays
@@ -555,9 +572,10 @@ def run_cross_topk(x, y, global_na=(), k=10, by="abs", scale_max=True, side="bot
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(L.icikt_cross_topk(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o), k, TOPK_BY[by],
-                             int(bool(scale_max)), *(ctypes.byref(v) if v is not None else None for v in lists),
-                             ctypes.byref(mx), ctypes.byref(t)))
+    check(getattr(L, "icikt_cross_topk" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
+                                                *dargs, k, TOPK_BY[by], int(bool(scale_max)),
+                                                *(ctypes.byref(v) if v is not None else None for v in lists),
+                                                ctypes.byref(mx), ctypes.byref(t)))
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 

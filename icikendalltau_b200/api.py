@@ -435,7 +435,9 @@ def ici_kendalltau_cross(x, y, global_na=(np.nan, np.inf, 0), perspective="globa
 
     min_abs_cor / max_pvalue (return_matrix=False) keep only the rows with abs(cor) >= min_abs_cor and
     pvalue <= max_pvalue, selected on the device (_lib.run_cross_edges) with the rules of ici_kendalltau's filtered
-    table; max_edges raises IciktError (ERR_LIMIT) when more pairs pass.  One GPU: n_gpus must be 1.
+    table; max_edges raises IciktError (ERR_LIMIT) when more pairs pass.  One GPU: n_gpus must be 1.  The same
+    results over several GPUs are _lib.run_cross(x, y, devices=[...]) and _lib.run_cross_edges(..., devices=[...]),
+    which return bit for bit what one GPU returns.
     """
     if n_gpus != 1:
         raise ValueError("the cross calls run on one GPU: n_gpus must be 1")
@@ -481,7 +483,8 @@ def ici_kendalltau_cross_topk(x, y, k, by="abs", side="x", global_na=(np.nan, np
     its best columns of x; "both": the two lists, e.g. for mutual nearest neighbours between two batches.  Ranking,
     padding and values are those of ici_kendalltau_topk over the Cx x Cy pairs; cor = raw / max(taumax over those
     pairs) if scale_max else raw.  The lists are selected on the device window by window (_lib.run_cross_topk) and
-    held there only for the requested sides.  One GPU: n_gpus must be 1.
+    held there only for the requested sides.  One GPU: n_gpus must be 1.  The same lists over several GPUs are
+    _lib.run_cross_topk(x, y, ..., devices=[...]), which returns bit for bit what one GPU returns.
 
     Returns a dict with key "x" and/or "y": per side the dict ici_kendalltau_topk returns (`index`, `neighbors` --
     names from the other matrix --, `cor`, `raw`, `pvalue`, `taumax`, `completeness`, `n_neighbors`, `max_taumax`,

@@ -1855,21 +1855,29 @@ struct WalkTotals {
   unsigned long long bits = 0;
 };
 
+// The upload of columns [c_lo, c_hi) of [X | Y] (y: Y of a cross call, from column s.C on, or null): X's part, then
+// Y's part.  X's CSC arrays occupy the plan's CSC buffers, which Y's overwrite (and may reallocate), so X's part is
+// expanded before Y's is uploaded; x_launches: that expansion's launches.
+static int upload_span(icikt_plan* p, const ColumnSource& s, const ColumnSource* y, int64_t c_lo, int64_t c_hi,
+                       int* x_launches) {
+  *x_launches = 0;
+  int rc = upload_columns(p, s, std::min(c_lo, s.C), std::min(c_hi, s.C));
+  if (rc != ICIKT_OK || !y || c_hi <= s.C) return rc;
+  *x_launches = expand_columns(p);
+  if (*x_launches < 0) return ICIKT_ERR_CUDA;
+  if (*x_launches > 0 && y->csc()) CK(cudaStreamSynchronize(p->stream));
+  rc = copy_columns_in(p, *y, std::max<int64_t>(c_lo - s.C, 0), c_hi - s.C, p->stream, s.C);
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[1], p->stream));
+  return ICIKT_OK;
+}
+
 // upload and K1 of the single-device filtered calls, ahead of their window walk.  A cross call passes Y as `y`: its
 // columns land behind X's, and K1 runs once over all columns of [X | Y].
 static int window_columns(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
                           const ColumnSource* y = nullptr) {
-  int rc = upload_columns(p, s, 0, s.C);
   int x_launches = 0;
-  if (rc == ICIKT_OK && y) {
-    // X's CSC arrays occupy the plan's CSC buffers, which Y's overwrite (and may reallocate): X is expanded first
-    x_launches = expand_columns(p);
-    if (x_launches < 0) return ICIKT_ERR_CUDA;
-    if (x_launches > 0 && y->csc()) CK(cudaStreamSynchronize(p->stream));
-    rc = copy_columns_in(p, *y, 0, y->C, p->stream, s.C);
-    if (rc != ICIKT_OK) return rc;
-    CK(cudaEventRecord(p->ev[1], p->stream));
-  }
+  int rc = upload_span(p, s, y, 0, p->C, &x_launches);
   if (rc == ICIKT_OK) rc = plan_columns_impl(p, global_na, n_global_na, 0, p->C, true);
   p->tm.n_launches += x_launches;
   return rc;
@@ -2174,6 +2182,30 @@ static void topk_fill_host(const TopkOut& out, int64_t C, int k, Held&& held, co
   }
 }
 
+// One side of a top-k result in the caller's arrays: rows [row0, row0 + cols) of the device lists.  `shift` is
+// subtracted from its partners once they are copied (a cross call's x side: plan column Cx + j becomes Y's index j);
+// raw: out.raw or the buffer topk_raw_buffer gave.
+struct TopkSide {
+  TopkOut out;
+  int64_t row0, cols;
+  int32_t shift;
+  std::vector<double> raw_own;
+  double* raw = nullptr;
+};
+
+// The host's part once every side's lists are in the caller's arrays: the partner shift, then topk_fill_host;
+// held(row): the entries of list row `row`.
+template <class Held>
+static void topk_sides_finish(std::vector<TopkSide>& sides, int k, Held&& held, bool scale, double M) {
+  for (TopkSide& sd : sides) {
+    auto side_held = [&](int64_t c) { return (int64_t)held(sd.row0 + c); };
+    if (sd.shift)
+      for (int64_t c = 0; c < sd.cols; ++c)
+        for (int64_t r = 0, h = side_held(c); r < h; ++r) sd.out.index[c * k + r] -= sd.shift;
+    topk_fill_host(sd.out, sd.cols, k, side_held, sd.raw, scale, M);
+  }
+}
+
 // The top-k call on one device: nothing comes back until the last window, then the lists are copied out once and
 // cor is formed with the final maximum.
 static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na, int k,
@@ -2424,14 +2456,9 @@ static int cross_plan(int64_t n, int64_t C, int64_t W, icikt_opts o, icikt_plan*
   return window_plan(g_cached_edges, n, C, W, o, out);
 }
 
-// icikt_cross_pairs on one device: per window, the results move off the plan's pair buffers into d_cres[b] on the
-// compute stream (the next window's K3 overwrites those buffers), and the host copies them from there into the
-// caller's arrays on the copy stream while the next window computes.
-static int cross_pair_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
-                              int32_t n_global_na, int64_t first, int64_t last, int64_t W, double* raw, double* pvalue,
-                              double* taumax, double* completeness, int32_t* status, double* max_taumax,
-                              icikt_timings* timings) {
-  int rc = ensure_walk_buffers(p);
+// the walk buffers of icikt_cross_pairs and its two result windows (kept with the plan)
+static int ensure_cross_buffers(icikt_plan* p) {
+  const int rc = ensure_walk_buffers(p);
   if (rc != ICIKT_OK) return rc;
   const size_t win = (size_t)p->P;  // the plan's pair buffers: W pairs and more
   for (int b = 0; b < 2; ++b)
@@ -2439,12 +2466,19 @@ static int cross_pair_windows(icikt_plan* p, const ColumnSource& sx, const Colum
       cudaGetLastError();
       return fail(ICIKT_ERR_ALLOC, "device allocation of the cross call's result windows failed");
     }
-  rc = window_columns(p, sx, global_na, n_global_na, &sy);
-  if (rc != ICIKT_OK) return rc;
+  return ICIKT_OK;
+}
+
+// icikt_cross_pairs' walk over pairs [first, last) of the Cx x Cy cross order, into caller arrays indexed from 0 =
+// first: per window, the results move off the plan's pair buffers into d_cres[b] on the compute stream (the next
+// window's K3 overwrites those buffers), and the host copies them from there into the caller's arrays on the copy
+// stream while the next window computes.
+static int cross_pair_walk(icikt_plan* p, int64_t Cx, int64_t Cy, int64_t first, int64_t last, int64_t W, double* raw,
+                           double* pvalue, double* taumax, double* completeness, int32_t* status, WalkTotals& tot,
+                           float& d2h_ms) {
+  const size_t win = (size_t)p->P;
   const double* d_field[4] = {p->d_tau, p->d_p, p->d_tm, p->d_comp};
   double* host_field[4] = {raw, pvalue, taumax, completeness};
-  WalkTotals tot;
-  float d2h_ms = 0.f;
   auto select = [&](int64_t, int b, const PairUnit*, int64_t, int64_t n_slots) -> int {
     double* to = reinterpret_cast<double*>(p->d_cres[b]);
     for (int f = 0; f < 4; ++f)
@@ -2470,7 +2504,20 @@ static int cross_pair_windows(icikt_plan* p, const ColumnSource& sx, const Colum
     d2h_ms += ev_ms(p->ev[6], p->ev[7]);
     return ICIKT_OK;
   };
-  rc = walk_windows(p, cross_order(sx.C, sy.C), first, last, W, tot, select, collect);
+  return walk_windows(p, cross_order(Cx, Cy), first, last, W, tot, select, collect);
+}
+
+// icikt_cross_pairs on one device
+static int cross_pair_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
+                              int32_t n_global_na, int64_t first, int64_t last, int64_t W, double* raw, double* pvalue,
+                              double* taumax, double* completeness, int32_t* status, double* max_taumax,
+                              icikt_timings* timings) {
+  int rc = ensure_cross_buffers(p);
+  if (rc == ICIKT_OK) rc = window_columns(p, sx, global_na, n_global_na, &sy);
+  if (rc != ICIKT_OK) return rc;
+  WalkTotals tot;
+  float d2h_ms = 0.f;
+  rc = cross_pair_walk(p, sx.C, sy.C, first, last, W, raw, pvalue, taumax, completeness, status, tot, d2h_ms);
   if (rc == ICIKT_OK) rc = finish_walk(p, tot, d2h_ms, timings);
   if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = max_of_bits(tot.bits);
@@ -2532,32 +2579,42 @@ static int cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, co
   return ICIKT_OK;
 }
 
-// icikt_cross_topk on one device: lists for the columns of the requested sides only, [c_lo, c_hi) of [X | Y] (X's
-// columns come first, so any choice of sides is one range); after the last window each side's rows of the lists go
-// to its caller arrays, and an x-side partner (a column Cx + j of the plan) becomes Y's index j.
+// The list rows of a cross top-k call, [c_lo, c_hi) of [X | Y] (X's columns come first, so any choice of sides is one
+// range), and its sides with their raw buffers: x_side rows from 0, y_side rows from Cx - c_lo.
+static int cross_topk_sides(const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, int64_t Cx, int64_t Cy,
+                            int k, int64_t* c_lo, int64_t* c_hi, std::vector<TopkSide>& sides) {
+  *c_lo = x_side ? 0 : Cx;
+  *c_hi = y_side ? Cx + Cy : Cx;
+  if (x_side) sides.push_back(TopkSide{TopkOut{x_side->index, x_side->n_neighbors, x_side->cor, x_side->raw,
+                                               x_side->pvalue, x_side->taumax, x_side->completeness},
+                                       0, Cx, (int32_t)Cx, {}, nullptr});
+  if (y_side) sides.push_back(TopkSide{TopkOut{y_side->index, y_side->n_neighbors, y_side->cor, y_side->raw,
+                                               y_side->pvalue, y_side->taumax, y_side->completeness},
+                                       Cx - *c_lo, Cy, 0, {}, nullptr});
+  for (TopkSide& sd : sides) {
+    const int rc = topk_raw_buffer(sd.out, sd.cols * k, sd.raw_own, &sd.raw);
+    if (rc != ICIKT_OK) return rc;
+  }
+  return ICIKT_OK;
+}
+
+// icikt_cross_topk on one device: lists for the columns of the requested sides only; after the last window each
+// side's rows of the lists go to its caller arrays, and an x-side partner (a column Cx + j of the plan) becomes Y's
+// index j.
 static int cross_topk_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
                               int32_t n_global_na, int k, int by, bool scale, int64_t W, const icikt_topk_lists* x_side,
                               const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings) {
   const int64_t Cx = sx.C, Cy = sy.C;
-  const int64_t c_lo = x_side ? 0 : Cx, c_hi = y_side ? Cx + Cy : Cx, L = c_hi - c_lo;
-  int rc = ensure_topk_buffers(p, W, k, L);
+  int64_t c_lo = 0, c_hi = 0;
+  std::vector<TopkSide> sides;
+  int rc = cross_topk_sides(x_side, y_side, Cx, Cy, k, &c_lo, &c_hi, sides);
+  const int64_t L = c_hi - c_lo;
+  if (rc == ICIKT_OK) rc = ensure_topk_buffers(p, W, k, L);
   if (rc == ICIKT_OK) rc = window_columns(p, sx, global_na, n_global_na, &sy);
   if (rc != ICIKT_OK) return rc;
   WalkTotals tot;
   rc = topk_walk(p, cross_order(Cx, Cy), c_lo, c_hi, k, by, 0, Cx * Cy, W, tot);
   if (rc != ICIKT_OK) return rc;
-  struct Side {
-    TopkOut out;
-    int64_t row0, cols;  // its first list row and its columns
-    int32_t shift;       // subtracted from its partners
-    std::vector<double> raw_own;
-    double* raw = nullptr;
-  };
-  std::vector<Side> sides;
-  if (x_side) sides.push_back(Side{TopkOut{x_side->index, x_side->n_neighbors, x_side->cor, x_side->raw, x_side->pvalue,
-                                           x_side->taumax, x_side->completeness}, 0, Cx, (int32_t)Cx, {}, nullptr});
-  if (y_side) sides.push_back(Side{TopkOut{y_side->index, y_side->n_neighbors, y_side->cor, y_side->raw, y_side->pvalue,
-                                           y_side->taumax, y_side->completeness}, Cx - c_lo, Cy, 0, {}, nullptr});
   std::vector<TopkCol> col;
   try {
     col.resize((size_t)L);
@@ -2567,9 +2624,8 @@ static int cross_topk_windows(icikt_plan* p, const ColumnSource& sx, const Colum
   CK(cudaEventRecord(p->ev[6], p->stream));
   rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)L, p->stream);
   const int64_t lk = L * k;
-  for (Side& sd : sides) {
+  for (TopkSide& sd : sides) {
     const int64_t ck = sd.cols * k, at = sd.row0 * k;
-    if (rc == ICIKT_OK) rc = topk_raw_buffer(sd.out, ck, sd.raw_own, &sd.raw);
     if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index, p->d_tidx + at, sizeof(int32_t) * (size_t)ck, p->stream);
     double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
     for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
@@ -2581,13 +2637,7 @@ static int cross_topk_windows(icikt_plan* p, const ColumnSource& sx, const Colum
   CK(cudaEventSynchronize(p->ev[7]));
   const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
   const double M = max_of_bits(tot.bits);
-  for (Side& sd : sides) {
-    auto held = [&](int64_t c) { return (int64_t)col[(size_t)(sd.row0 + c)].n; };
-    if (sd.shift)
-      for (int64_t c = 0; c < sd.cols; ++c)
-        for (int64_t r = 0, h = held(c); r < h; ++r) sd.out.index[c * k + r] -= sd.shift;
-    topk_fill_host(sd.out, sd.cols, k, held, sd.raw, scale, M);
-  }
+  topk_sides_finish(sides, k, [&](int64_t row) { return col[(size_t)row].n; }, scale, M);
   rc = finish_walk(p, tot, d2h_ms, timings);
   if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = M;
@@ -2759,23 +2809,25 @@ namespace {
 // NVSwitch), device k uploads only its slice of the columns over its own PCIe link, runs K1 on that
 // slice and pulls the other slices of the per-column TABLES from its peers (an all-gather by peer
 // copies: K1 is not replicated and the raw matrix never travels between devices); otherwise every
-// device uploads the whole matrix and preprocesses all columns.
+// device uploads the whole matrix and preprocesses all columns.  A cross call's job holds [X | Y]: src is X, y is Y
+// (placed from column src.C on), C = Cx + Cy, and the slices cover pairs [first, first + ptot) of the cross order.
 struct MultiJob {
   ColumnSource src;
+  const ColumnSource* y = nullptr;
   int64_t n, C;
   const double* global_na;
   int32_t n_global_na;
   icikt_opts base;
   const int32_t* devices;
   int n_devices;
-  int64_t ptot;
+  int64_t first = 0, ptot;
   bool peers_ok = false;  // every pair of distinct ordinals has peer access
   bool gather = false;    // sharded K1 + peer gather of the tables
   HostBarrier barrier;
   std::vector<icikt_plan*> peer_plan;
   explicit MultiJob(int nd) : n_devices(nd), barrier(nd), peer_plan((size_t)nd, nullptr) {}
   int device_of(int k) const { return devices ? devices[k] : k; }
-  int64_t pair_lo(int k) const { return ptot * k / n_devices; }  // slices differ by at most one pair
+  int64_t pair_lo(int k) const { return first + ptot * k / n_devices; }  // slices differ by at most one pair
   int64_t col_lo(int k) const { return C * k / n_devices; }
 };
 
@@ -2791,8 +2843,10 @@ void multi_probe_peers(MultiJob& J) {
       if (cudaDeviceCanAccessPeer(&ok, da, db) != cudaSuccess || !ok) J.peers_ok = false;
     }
   cudaGetLastError();
-  J.gather = J.n_devices >= 2 && distinct && J.peers_ok && J.C >= J.n_devices && J.ptot >= J.n_devices &&
-             !std::getenv("ICIKT_NO_PEER_GATHER");
+  // ICIKT_FORCE_PEER_GATHER: repeated ordinals take gather mode too (a same-device peer copy is a device-to-device
+  // copy), so that one GPU runs the sharded column phase
+  J.gather = J.n_devices >= 2 && (distinct || std::getenv("ICIKT_FORCE_PEER_GATHER")) && J.peers_ok &&
+             J.C >= J.n_devices && J.ptot >= J.n_devices && !std::getenv("ICIKT_NO_PEER_GATHER");
 }
 
 int enable_peers(const MultiJob& J, int k) {
@@ -2807,17 +2861,21 @@ int enable_peers(const MultiJob& J, int k) {
 
 // The column phase of worker k on its plan p (rc: how getting the plan went): sharded K1 and the peer gather of the
 // tables in gather mode, otherwise the upload and K1 of all columns (skipped when the worker has no pairs).  In
-// gather mode every worker passes both barriers whatever happened to it, so nobody is left waiting.
+// gather mode every worker passes both barriers whatever happened to it, so nobody is left waiting.  A cross job's
+// columns are those of [X | Y]: a shard that straddles column Cx uploads X's part, then Y's (upload_span).
 int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
   const int64_t cnt = J.pair_lo(k + 1) - J.pair_lo(k);
   if (!J.gather) {
-    if (cnt <= 0) return rc;
-    if (rc == ICIKT_OK) rc = J.src.csc() ? upload_columns(p, J.src, 0, J.C) : icikt_plan_upload(p, J.src.data, J.src.ld);
+    if (cnt <= 0 || rc != ICIKT_OK) return rc;
+    if (J.y) return window_columns(p, J.src, J.global_na, J.n_global_na, J.y);
+    rc = J.src.csc() ? upload_columns(p, J.src, 0, J.C) : icikt_plan_upload(p, J.src.data, J.src.ld);
     if (rc == ICIKT_OK) rc = icikt_plan_columns(p, J.global_na, J.n_global_na);
     return rc;
   }
-  if (rc == ICIKT_OK) rc = upload_columns(p, J.src, J.col_lo(k), J.col_lo(k + 1));
+  int x_launches = 0;
+  if (rc == ICIKT_OK) rc = upload_span(p, J.src, J.y, J.col_lo(k), J.col_lo(k + 1), &x_launches);
   if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
+  if (rc == ICIKT_OK) p->tm.n_launches += x_launches;
   if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "column slice");
   J.peer_plan[(size_t)k] = (rc == ICIKT_OK) ? p : nullptr;
   J.barrier.wait();  // every slice of the tables is complete on its device
@@ -3100,6 +3158,71 @@ int window_multi_worker(MultiJob& J, int k, icikt_plan** out) {
   return rc;
 }
 
+// walk(order) with the pair order of J's walk: the cross order of a cross job, the combn order of p otherwise
+template <class Walk>
+int with_order(const MultiJob& J, const icikt_plan* p, Walk&& walk) {
+  return J.y ? walk(cross_order(J.src.C, J.y->C)) : walk(combn_order(p));
+}
+
+// The filtered call over the devices of J, its arguments checked: every worker walks its slice against the shared
+// EdgeHeld, then the rows are joined in worker order (the slices are contiguous and in order, so are the rows) and
+// edge_result trims them with the final maximum.
+int edges_multi_run(MultiJob& J, const icikt_edge_filter& f, icikt_edges* res, double* max_taumax,
+                    icikt_timings* timings) {
+  const int n_devices = J.n_devices;
+  std::vector<MultiWork> work((size_t)n_devices);
+  std::vector<std::vector<EdgeRow>> rows((size_t)n_devices);
+  std::vector<unsigned long long> bits((size_t)n_devices, 0);
+  EdgeHeld held;
+  {
+    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+    multi_probe_peers(J);
+    std::vector<std::thread> threads;
+    for (int k = 0; k < n_devices; ++k) {
+      threads.emplace_back([&, k]() {
+        MultiWork& w = work[(size_t)k];
+        icikt_plan* p = nullptr;
+        w.rc = window_multi_worker(J, k, &p);
+        const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
+        if (w.rc == ICIKT_OK && hi > lo) {
+          WalkTotals tot;
+          float d2h_ms = 0.f;
+          w.rc = ensure_edge_buffers(p, p->P);
+          if (w.rc == ICIKT_OK)
+            w.rc = with_order(J, p, [&](const auto& order) {
+              return edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
+            });
+          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
+          bits[(size_t)k] = tot.bits;
+        }
+        if (w.rc != ICIKT_OK) {
+          w.err = g_err;  // thread-local message of this worker
+          drop_window_plan(g_cached_wmulti[k]);
+        }
+      });
+    }
+    for (auto& t : threads) t.join();
+  }
+  int rc = multi_collect(work, nullptr, timings);
+  if (rc != ICIKT_OK) return rc;
+  size_t total = 0;
+  for (const auto& r : rows) total += r.size();
+  try {
+    res->rows.reserve(total);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the selected rows");
+  }
+  for (auto& r : rows) {
+    res->rows.insert(res->rows.end(), r.begin(), r.end());
+    std::vector<EdgeRow>().swap(r);
+  }
+  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  rc = edge_result(res, f, M);
+  if (rc != ICIKT_OK) return rc;
+  if (max_taumax) *max_taumax = M;
+  return ICIKT_OK;
+}
+
 int edges_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
                      const icikt_opts* opts, const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
                      icikt_edges** out, double* max_taumax, icikt_timings* timings) {
@@ -3120,67 +3243,21 @@ int edges_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* 
   if (rc != ICIKT_OK) return rc;
   std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
   if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
-  const icikt_edge_filter& f = *filter;
-  std::vector<MultiWork> work((size_t)n_devices);
-  std::vector<std::vector<EdgeRow>> rows((size_t)n_devices);
-  std::vector<unsigned long long> bits((size_t)n_devices, 0);
-  EdgeHeld held;
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
-    multi_probe_peers(J);
-    std::vector<std::thread> threads;
-    for (int k = 0; k < n_devices; ++k) {
-      threads.emplace_back([&, k]() {
-        MultiWork& w = work[(size_t)k];
-        icikt_plan* p = nullptr;
-        w.rc = window_multi_worker(J, k, &p);
-        const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
-        if (w.rc == ICIKT_OK && hi > lo) {
-          WalkTotals tot;
-          float d2h_ms = 0.f;
-          w.rc = ensure_edge_buffers(p, p->P);
-          if (w.rc == ICIKT_OK) w.rc = edge_walk(p, combn_order(p), f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
-          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
-          bits[(size_t)k] = tot.bits;
-        }
-        if (w.rc != ICIKT_OK) {
-          w.err = g_err;  // thread-local message of this worker
-          drop_window_plan(g_cached_wmulti[k]);
-        }
-      });
-    }
-    for (auto& t : threads) t.join();
-  }
-  rc = multi_collect(work, nullptr, timings);
+  rc = edges_multi_run(J, *filter, res.get(), max_taumax, timings);
   if (rc != ICIKT_OK) return rc;
-  // the slices are contiguous and in worker order: so are the rows
-  size_t total = 0;
-  for (const auto& r : rows) total += r.size();
-  try {
-    res->rows.reserve(total);
-  } catch (const std::bad_alloc&) {
-    return fail(ICIKT_ERR_ALLOC, "out of host memory for the selected rows");
-  }
-  for (auto& r : rows) {
-    res->rows.insert(res->rows.end(), r.begin(), r.end());
-    std::vector<EdgeRow>().swap(r);
-  }
-  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
-  rc = edge_result(res.get(), f, M);
-  if (rc != ICIKT_OK) return rc;
-  if (max_taumax) *max_taumax = M;
   *out = res.release();
   return ICIKT_OK;
 }
 
-// Worker k's block of columns [col_lo(k), col_lo(k + 1)) of the merged lists: the merge kernel reads every device's
-// lists in place, and the block goes straight into the caller's arrays at c_lo * k (raw: out.raw or the host
-// buffer for cor); held[c] receives column c's entries.  tm: the merge and its copies become d2h_ms.
-int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<icikt_plan*>& plans, int K, int by,
-                     const TopkOut& out, double* raw, int32_t* held, icikt_timings& tm) {
-  const int64_t c_lo = J.col_lo(k), c_hi = J.col_lo(k + 1);
-  if (c_hi <= c_lo) return ICIKT_OK;
-  const size_t blk = (size_t)(c_hi - c_lo) * (size_t)K, off = (size_t)c_lo * (size_t)K;
+// Worker k's block of list rows [L*k/N, L*(k+1)/N) of the merged lists (L rows: the columns of an all-pairs call,
+// the requested sides of a cross call): the merge kernel reads every device's lists in place, and the block goes
+// straight into the caller's arrays of every side it covers (one block may hold rows of both sides of a cross
+// call); held[r] receives row r's entries.  tm: the merge and its copies become d2h_ms.
+int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<icikt_plan*>& plans, int64_t L, int K,
+                     int by, const std::vector<TopkSide>& sides, int32_t* held, icikt_timings& tm) {
+  const int64_t r_lo = L * k / J.n_devices, r_hi = L * (k + 1) / J.n_devices;
+  if (r_hi <= r_lo) return ICIKT_OK;
+  const size_t blk = (size_t)(r_hi - r_lo) * (size_t)K;
   int rc = ensure_merge_buffers(p, blk);
   if (rc != ICIKT_OK) return rc;
   TopkDeviceMerge m{};
@@ -3190,9 +3267,9 @@ int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<
     m.idx[j] = plans[(size_t)j]->d_tidx;
     m.list[j] = plans[(size_t)j]->d_tlist;
   }
-  m.C = J.C;
-  m.c_lo = c_lo;
-  m.c_hi = c_hi;
+  m.C = L;  // the lists' rows: the kernel's columns
+  m.c_lo = r_lo;
+  m.c_hi = r_hi;
   m.k = K;
   m.by = by;
   m.n = p->d_mn;
@@ -3202,17 +3279,82 @@ int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<
   const int l = launch_topk_device_merge(m, p->stream);
   if (l < 0) return launch_fail("top-k device merge kernel");
   tm.n_launches += l;
-  rc = staged_copy_out(p, held + c_lo, p->d_mn, sizeof(int32_t) * (size_t)(c_hi - c_lo), p->stream);
-  if (rc == ICIKT_OK) rc = staged_copy_out(p, out.index + off, p->d_midx, sizeof(int32_t) * blk, p->stream);
-  double* host_field[4] = {raw, out.pvalue, out.taumax, out.completeness};
-  for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
-    if (host_field[f]) rc = staged_copy_out(p, host_field[f] + off, p->d_mlist + f * blk, sizeof(double) * blk, p->stream);
+  rc = staged_copy_out(p, held + r_lo, p->d_mn, sizeof(int32_t) * (size_t)(r_hi - r_lo), p->stream);
+  for (const TopkSide& sd : sides) {
+    const int64_t lo = std::max(r_lo, sd.row0), hi = std::min(r_hi, sd.row0 + sd.cols);
+    if (hi <= lo) continue;
+    const size_t len = (size_t)(hi - lo) * (size_t)K, from = (size_t)(lo - r_lo) * (size_t)K,
+                 to = (size_t)(lo - sd.row0) * (size_t)K;
+    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index + to, p->d_midx + from, sizeof(int32_t) * len, p->stream);
+    double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
+    for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
+      if (host_field[f])
+        rc = staged_copy_out(p, host_field[f] + to, p->d_mlist + f * blk + from, sizeof(double) * len, p->stream);
+  }
   if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[7], p->stream));
   CK(cudaEventSynchronize(p->ev[7]));
   tm.d2h_ms = ev_ms(p->ev[6], p->ev[7]);
   tm.total_ms = ev_ms(p->ev[0], p->ev[7]);
   cudaGetLastError();
+  return ICIKT_OK;
+}
+
+// The top-k call over the devices of J, its arguments checked and peer access found: every worker keeps the lists of
+// rows [c_lo, c_hi) (columns of the plan) for its slice; after a barrier, worker k merges its block of rows into
+// the sides' arrays; then the host shifts the partners and pads (topk_sides_finish).
+int topk_multi_run(MultiJob& J, int K, int by, bool scale, int64_t c_lo, int64_t c_hi, std::vector<TopkSide>& sides,
+                   double* max_taumax, icikt_timings* timings) {
+  const int n_devices = J.n_devices;
+  const int64_t L = c_hi - c_lo;
+  std::vector<int32_t> held;
+  try {
+    held.resize((size_t)L);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
+  }
+  std::vector<MultiWork> work((size_t)n_devices);
+  std::vector<unsigned long long> bits((size_t)n_devices, 0);
+  std::vector<icikt_plan*> plans((size_t)n_devices, nullptr);
+  {
+    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+    std::vector<std::thread> threads;
+    for (int k = 0; k < n_devices; ++k) {
+      threads.emplace_back([&, k]() {
+        MultiWork& w = work[(size_t)k];
+        icikt_plan* p = nullptr;
+        w.rc = window_multi_worker(J, k, &p);
+        if (w.rc == ICIKT_OK) {
+          WalkTotals tot;
+          w.rc = ensure_topk_buffers(p, p->P, K, L);
+          if (w.rc == ICIKT_OK)
+            w.rc = with_order(J, p, [&](const auto& order) {
+              return topk_walk(p, order, c_lo, c_hi, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
+            });
+          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, 0.f, &w.tm);
+          bits[(size_t)k] = tot.bits;
+        }
+        plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
+        J.barrier.wait();  // every device's lists are complete
+        bool all_ok = true;
+        for (int j = 0; j < n_devices; ++j) all_ok = all_ok && plans[(size_t)j] != nullptr;
+        if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to select its lists");
+        if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
+        if (w.rc == ICIKT_OK) w.rc = topk_merge_block(J, k, p, plans, L, K, by, sides, held.data(), w.tm);
+        J.barrier.wait();  // nobody's lists are freed (or reused) before every block has been merged
+        if (w.rc != ICIKT_OK) {
+          w.err = g_err;
+          drop_window_plan(g_cached_wmulti[k]);
+        }
+      });
+    }
+    for (auto& t : threads) t.join();
+  }
+  const int rc = multi_collect(work, nullptr, timings);
+  if (rc != ICIKT_OK) return rc;
+  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  topk_sides_finish(sides, K, [&](int64_t row) { return held[(size_t)row]; }, scale, M);
+  if (max_taumax) *max_taumax = M;
   return ICIKT_OK;
 }
 
@@ -3239,45 +3381,74 @@ int topk_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* g
     o.device = J.device_of(0);
     return all_pairs_topk(s, n, C, global_na, n_global_na, &o, K, by, scale_max, out, max_taumax, timings);
   }
-  const int64_t ck = C * K;
-  std::vector<double> raw_own;
-  double* raw = nullptr;
-  rc = topk_raw_buffer(out, ck, raw_own, &raw);
+  std::vector<TopkSide> sides(1);
+  sides[0].out = out;
+  sides[0].row0 = 0;
+  sides[0].cols = C;
+  sides[0].shift = 0;
+  rc = topk_raw_buffer(out, C * K, sides[0].raw_own, &sides[0].raw);
   if (rc != ICIKT_OK) return rc;
-  std::vector<int32_t> held;
-  try {
-    held.resize((size_t)C);
-  } catch (const std::bad_alloc&) {
-    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
+  return topk_multi_run(J, K, by, scale_max != 0, 0, C, sides, max_taumax, timings);
+}
+
+// ---- the cross calls over several devices: the cross order (of the call's range) sliced as above over the
+// Cx + Cy columns of [X | Y]
+
+// A cross job over pairs [first, last) of the cross order, its arguments checked.  The window plans hold W pairs of
+// a slice: the call's pair range is the job's, not theirs.
+void cross_job(MultiJob& J, const ColumnSource& sx, const ColumnSource& sy, int64_t n, const double* global_na,
+               int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int64_t first, int64_t last) {
+  J.src = sx; J.y = &sy; J.n = n; J.C = sx.C + sy.C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.base.pair_lo = J.base.pair_hi = 0;
+  J.first = first; J.ptot = last - first;
+}
+
+int cross_pairs_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                      double* raw, double* pvalue, double* taumax, double* completeness, int32_t* status,
+                      double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  ColumnSource sx, sy;
+  int rc = check_cross_args(x, y, n, global_na, n_global_na, o, true, &sx, &sy);
+  if (rc == ICIKT_OK && !raw) rc = fail(ICIKT_ERR_BAD_ARG, "raw is NULL");
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  const int64_t first = o.pair_lo, last = (o.pair_hi == 0) ? sx.C * sy.C : o.pair_hi;
+  MultiJob J(n_devices);
+  cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, first, last);
+  if (n_devices == 1 || last == first) {
+    o.device = J.device_of(0);
+    return cross_pairs(x, y, n, global_na, n_global_na, &o, raw, pvalue, taumax, completeness, status, max_taumax,
+                       timings);
   }
+  rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
   std::vector<MultiWork> work((size_t)n_devices);
   std::vector<unsigned long long> bits((size_t)n_devices, 0);
-  std::vector<icikt_plan*> plans((size_t)n_devices, nullptr);
   {
     std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+    multi_probe_peers(J);
     std::vector<std::thread> threads;
     for (int k = 0; k < n_devices; ++k) {
       threads.emplace_back([&, k]() {
         MultiWork& w = work[(size_t)k];
         icikt_plan* p = nullptr;
         w.rc = window_multi_worker(J, k, &p);
-        if (w.rc == ICIKT_OK) {
+        const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1), off = lo - first;
+        if (w.rc == ICIKT_OK && hi > lo) {
           WalkTotals tot;
-          w.rc = ensure_topk_buffers(p, p->P, K, J.C);
-          if (w.rc == ICIKT_OK) w.rc = topk_walk(p, combn_order(p), 0, J.C, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
-          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, 0.f, &w.tm);
+          float d2h_ms = 0.f;
+          w.rc = ensure_cross_buffers(p);
+          if (w.rc == ICIKT_OK)
+            w.rc = cross_pair_walk(p, sx.C, sy.C, lo, hi, p->P, raw + off, pvalue ? pvalue + off : nullptr,
+                                   taumax ? taumax + off : nullptr, completeness ? completeness + off : nullptr,
+                                   status ? status + off : nullptr, tot, d2h_ms);
+          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
           bits[(size_t)k] = tot.bits;
         }
-        plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
-        J.barrier.wait();  // every device's lists are complete
-        bool all_ok = true;
-        for (int j = 0; j < n_devices; ++j) all_ok = all_ok && plans[(size_t)j] != nullptr;
-        if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to select its lists");
-        if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
-        if (w.rc == ICIKT_OK) w.rc = topk_merge_block(J, k, p, plans, K, by, out, raw, held.data(), w.tm);
-        J.barrier.wait();  // nobody's lists are freed (or reused) before every block has been merged
         if (w.rc != ICIKT_OK) {
-          w.err = g_err;
+          w.err = g_err;  // thread-local message of this worker
           drop_window_plan(g_cached_wmulti[k]);
         }
       });
@@ -3286,10 +3457,70 @@ int topk_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* g
   }
   rc = multi_collect(work, nullptr, timings);
   if (rc != ICIKT_OK) return rc;
-  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
-  topk_fill_host(out, C, K, [&](int64_t c) { return (int64_t)held[(size_t)c]; }, raw, scale_max != 0, M);
-  if (max_taumax) *max_taumax = M;
+  if (max_taumax) *max_taumax = max_of_bits(*std::max_element(bits.begin(), bits.end()));
   return ICIKT_OK;
+}
+
+int cross_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                      const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  ColumnSource sx, sy;
+  int rc = check_filter_args(filter, out);
+  if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  MultiJob J(n_devices);
+  cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
+  if (n_devices == 1) {
+    o.device = J.device_of(0);
+    return cross_edges(x, y, n, global_na, n_global_na, &o, filter, out, max_taumax, timings);
+  }
+  rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
+  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
+  res->j_offset = (int32_t)sx.C;
+  rc = edges_multi_run(J, *filter, res.get(), max_taumax, timings);
+  if (rc != ICIKT_OK) return rc;
+  *out = res.release();
+  return ICIKT_OK;
+}
+
+int cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                     int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices, int32_t K,
+                     int32_t by, int32_t scale_max, const icikt_topk_lists* x_side, const icikt_topk_lists* y_side,
+                     double* max_taumax, icikt_timings* timings) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  int rc = check_k_by(K, by);
+  if (rc != ICIKT_OK) return rc;
+  if (!x_side && !y_side) return fail(ICIKT_ERR_BAD_ARG, "x_side and y_side are both NULL");
+  if ((x_side && !x_side->index) || (y_side && !y_side->index))
+    return fail(ICIKT_ERR_BAD_ARG, x_side && !x_side->index ? "x_side->index is NULL" : "y_side->index is NULL");
+  ColumnSource sx, sy;
+  rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  MultiJob J(n_devices);
+  cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
+  rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  {
+    std::lock_guard<std::mutex> lock(g_cache_mu);
+    multi_probe_peers(J);
+  }
+  if (n_devices == 1 || !J.peers_ok) {
+    // one device, or devices that cannot read each other's lists: the single-device call
+    o.device = J.device_of(0);
+    return cross_topk(x, y, n, global_na, n_global_na, &o, K, by, scale_max, x_side, y_side, max_taumax, timings);
+  }
+  int64_t c_lo = 0, c_hi = 0;
+  std::vector<TopkSide> sides;
+  rc = cross_topk_sides(x_side, y_side, sx.C, sy.C, K, &c_lo, &c_hi, sides);
+  if (rc != ICIKT_OK) return rc;
+  return topk_multi_run(J, K, by, scale_max != 0, c_lo, c_hi, sides, max_taumax, timings);
 }
 
 }  // namespace
@@ -3378,6 +3609,29 @@ int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx,
   return topk_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices, n_devices, k,
                          by, scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness},
                          max_taumax, timings);
+}
+
+int icikt_cross_pairs_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                            double* raw, double* pvalue, double* taumax, double* completeness, int32_t* status,
+                            double* max_taumax, icikt_timings* timings) {
+  return cross_pairs_multi(x, y, n, global_na, n_global_na, opts, devices, n_devices, raw, pvalue, taumax, completeness,
+                           status, max_taumax, timings);
+}
+
+int icikt_cross_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                            const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                            icikt_timings* timings) {
+  return cross_edges_multi(x, y, n, global_na, n_global_na, opts, devices, n_devices, filter, out, max_taumax, timings);
+}
+
+int icikt_cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                           int32_t k, int32_t by, int32_t scale_max, const icikt_topk_lists* x_side,
+                           const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings) {
+  return cross_topk_multi(x, y, n, global_na, n_global_na, opts, devices, n_devices, k, by, scale_max, x_side, y_side,
+                          max_taumax, timings);
 }
 
 int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,

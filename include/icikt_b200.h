@@ -415,6 +415,47 @@ int icikt_cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, cons
                      const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
                      icikt_timings* timings);
 
+/* ---- the cross calls over several GPUs of one box in ONE call, as the filtered all-pairs multi calls above.  The
+ * cross order (of [pair_lo, pair_hi) for icikt_cross_pairs_multi) is sliced over the devices, and device k walks its
+ * slice in windows of min(ICIKT_EDGE_WINDOW, slice) pairs.  The columns are prepared as in icikt_all_pairs_multi
+ * over the Cx + Cy columns of [X | Y]: sharded K1 + peer gather of the tables when every pair of distinct devices has
+ * peer access (device k uploads and preprocesses its share of [X | Y], X's part, Y's part or both), otherwise every
+ * device uploads X and Y and preprocesses all columns.
+ *   Pairs: device k copies the results of its slice straight into the caller's arrays, at its offset from pair_lo.
+ *   Edges: as icikt_all_pairs_edges_multi; rows are joined in slice order, which is cross order.
+ *   Top-k: every device keeps the lists of the requested sides (rows [c_lo, c_hi) of [X | Y], L = c_hi - c_lo) for
+ *   its slice; then device k merges rows [L*k/N, L*(k+1)/N) of all devices' lists, reading them through peer access,
+ *   and copies them straight into x_side and / or y_side (a block may hold rows of both).
+ *
+ *   - Same result as one device: every output (the per-pair arrays, status, rows with their order and fields, cor,
+ *     max_taumax, index, n_neighbors, the padding, what icikt_edges_copy returns: j as Y's own index) is bit for bit
+ *     that of the matching single-device cross call with the same arguments.
+ *   - devices == NULL means ordinals 0..n_devices-1; repeated ordinals are allowed; 1 <= n_devices <= 16.
+ *     opts->device is ignored.
+ *   - Refused with ICIKT_ERR_BAD_ARG before any device is touched: whatever the single-device cross call refuses
+ *     (with the same messages, CSC ones naming the matrix and the column), and n_devices out of range.
+ *   - pair_lo / pair_hi: icikt_cross_pairs_multi takes them as icikt_cross_pairs does (the arrays are indexed from
+ *     0 = pair_lo); the edges and top-k calls refuse them.
+ *   - Peer access: the pairs and edges calls need none.  The top-k call needs it between distinct devices; without
+ *     it it runs icikt_cross_topk on devices[0].  With n_devices == 1 each call is its single-device call on
+ *     devices[0].
+ *   - max_edges: as icikt_all_pairs_edges_multi (the rows held are counted over all devices; once one device crosses
+ *     the limit, the others stop at their next window boundary).
+ *   - timings (may be NULL): the slowest device's figures, n_launches summed over the devices; for top-k, d2h_ms is
+ *     the merge of the device's block with its copy out. */
+int icikt_cross_pairs_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                            double* raw, double* pvalue, double* taumax, double* completeness, int32_t* status,
+                            double* max_taumax, icikt_timings* timings);
+int icikt_cross_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                            const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                            icikt_timings* timings);
+int icikt_cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                           int32_t k, int32_t by, int32_t scale_max, const icikt_topk_lists* x_side,
+                           const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings);
+
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
  * pay the copies.  A plan is bound to one device and is not thread-safe.            */
