@@ -1464,14 +1464,22 @@ static bool want_staged(int64_t n, int64_t C, const icikt_opts& o, bool all_pair
 // One cached plan for the one-shot entry points (all-pairs shape only).
 static icikt_plan* g_cached = nullptr;
 static icikt_plan* g_cached_multi[64] = {};  // one slot per worker of icikt_all_pairs_multi
-static icikt_plan* g_cached_edges = nullptr;    // the filtered call's (its pair buffers hold one window)
-static icikt_plan* g_cached_wmulti[kMaxMatrixDevices] = {};  // one slot per worker of the filtered calls' multi twins
+static icikt_plan* g_cached_edges = nullptr;    // a windowed call's on one device (its pair buffers hold one window)
+static icikt_plan* g_cached_wmulti[kMaxMatrixDevices] = {};  // one slot per worker of a windowed call on several
 static std::mutex g_cache_mu;
 
 static bool cache_matches(const icikt_plan* p, int64_t n, int64_t C, const icikt_opts& o, bool staged) {
   return p && p->staged == staged && p->n == n && p->C == C && p->opts.device == o.device && p->opts.kernel == o.kernel &&
          p->opts.include_diag == o.include_diag && p->opts.pair_lo == o.pair_lo &&
          p->opts.pair_hi == o.pair_hi && p->want_counts == (o.want_counts != 0);
+}
+
+// a cached plan taken by a call: the options that do not shape the plan are the call's
+static void reuse_plan(icikt_plan* p, const icikt_opts& o) {
+  p->opts.perspective = o.perspective;
+  p->opts.alternative = o.alternative;
+  p->opts.continuity = o.continuity;
+  p->opts.na_inf = o.na_inf;
 }
 
 struct MatrixOut {  // the download step of one_shot as matrices instead of per-pair arrays
@@ -1499,10 +1507,7 @@ static int one_shot(const ColumnSource& s, int64_t n, int64_t C, const double* g
   if (cacheable && cache_matches(g_cached, n, C, o, staged) &&
       (o.perspective != ICIKT_PERSPECTIVE_COMPLETE || g_cached->d_pw)) {
     p = g_cached;
-    p->opts.perspective = o.perspective;
-    p->opts.alternative = o.alternative;
-    p->opts.continuity = o.continuity;
-    p->opts.na_inf = o.na_inf;
+    reuse_plan(p, o);
   } else {
     if (cacheable && g_cached) { icikt_plan_destroy(g_cached); g_cached = nullptr; }
     rc = plan_create_impl(&p, n, C, pi, pj, P, &o, staged);
@@ -1872,8 +1877,8 @@ static int upload_span(icikt_plan* p, const ColumnSource& s, const ColumnSource*
   return ICIKT_OK;
 }
 
-// upload and K1 of the single-device filtered calls, ahead of their window walk.  A cross call passes Y as `y`: its
-// columns land behind X's, and K1 runs once over all columns of [X | Y].
+// upload and K1 of all columns on one device (the column phase of a multi-device job without peer gather).  A cross
+// job passes Y as `y`: its columns land behind X's, and K1 runs once over all columns of [X | Y].
 static int window_columns(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
                           const ColumnSource* y = nullptr) {
   int x_launches = 0;
@@ -2081,28 +2086,6 @@ static int edge_result(icikt_edges* res, const icikt_edge_filter& f, double M) {
   return ICIKT_OK;
 }
 
-// The filtered call on one device: upload, K1, the walk over the whole pair order, the final trim.  y: Y of a cross
-// call (the cross order), or null (combn order).
-static int edge_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na,
-                        const icikt_edge_filter& f, int64_t ptot, int64_t W, icikt_edges* res, double* max_taumax,
-                        icikt_timings* timings, const ColumnSource* y = nullptr) {
-  int rc = ensure_edge_buffers(p, W);
-  if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na, y);
-  if (rc != ICIKT_OK) return rc;
-  WalkTotals tot;
-  float d2h_ms = 0.f;
-  EdgeHeld held;
-  rc = y ? edge_walk(p, cross_order(s.C, y->C), f, 0, ptot, W, res->rows, held, tot, d2h_ms)
-         : edge_walk(p, combn_order(p), f, 0, ptot, W, res->rows, held, tot, d2h_ms);
-  if (rc != ICIKT_OK) return rc;
-  const double M = max_of_bits(tot.bits);
-  rc = edge_result(res, f, M);
-  if (rc == ICIKT_OK) rc = finish_walk(p, tot, d2h_ms, timings);
-  if (rc != ICIKT_OK) return rc;
-  if (max_taumax) *max_taumax = M;
-  return ICIKT_OK;
-}
-
 // The top-k call: per window, the top-k selection merges the window's candidates into the lists on the device;
 // nothing comes back until the last window, then the lists are copied out once and cor is formed with the
 // final maximum.
@@ -2206,57 +2189,14 @@ static void topk_sides_finish(std::vector<TopkSide>& sides, int k, Held&& held, 
   }
 }
 
-// The top-k call on one device: nothing comes back until the last window, then the lists are copied out once and
-// cor is formed with the final maximum.
-static int topk_windows(icikt_plan* p, const ColumnSource& s, const double* global_na, int32_t n_global_na, int k,
-                        int by, bool scale, int64_t ptot, int64_t W, const TopkOut& out, double* max_taumax,
-                        icikt_timings* timings) {
-  int rc = ensure_topk_buffers(p, W, k, p->C);
-  if (rc == ICIKT_OK) rc = window_columns(p, s, global_na, n_global_na);
-  if (rc != ICIKT_OK) return rc;
-  const int64_t C = p->C, ck = C * k;
-  WalkTotals tot;
-  rc = topk_walk(p, combn_order(p), 0, C, k, by, 0, ptot, W, tot);
-  if (rc != ICIKT_OK) return rc;
-  // the lists, once
-  std::vector<TopkCol> col;
-  std::vector<double> raw_own;
-  double* raw = nullptr;
-  try {
-    col.resize((size_t)C);
-  } catch (const std::bad_alloc&) {
-    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
-  }
-  rc = topk_raw_buffer(out, ck, raw_own, &raw);
-  if (rc != ICIKT_OK) return rc;
-  CK(cudaEventRecord(p->ev[6], p->stream));
-  rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)C, p->stream);
-  if (rc == ICIKT_OK) rc = staged_copy_out(p, out.index, p->d_tidx, sizeof(int32_t) * (size_t)ck, p->stream);
-  double* host_field[4] = {raw, out.pvalue, out.taumax, out.completeness};
-  for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
-    if (host_field[f]) rc = staged_copy_out(p, host_field[f], p->d_tlist + f * ck, sizeof(double) * (size_t)ck, p->stream);
-  if (rc != ICIKT_OK) return rc;
-  CK(cudaEventRecord(p->ev[7], p->stream));
-  CK(cudaEventSynchronize(p->ev[7]));
-  const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
-  const double M = max_of_bits(tot.bits);
-  topk_fill_host(out, C, k, [&](int64_t c) { return (int64_t)col[(size_t)c].n; }, raw, scale, M);
-  rc = finish_walk(p, tot, d2h_ms, timings);
-  if (rc != ICIKT_OK) return rc;
-  if (max_taumax) *max_taumax = M;
-  return ICIKT_OK;
-}
 #undef ECK
 
-// The plan of the filtered calls (cached in `slot`: g_cached_edges, or a worker's of the multi-device twins; the
-// caller holds g_cache_mu): pair buffers of one window of W pairs.
+// The plan of the windowed calls (cached in `slot`, see window_slots; the caller holds g_cache_mu): pair buffers of
+// one window of W pairs.
 static int window_plan(icikt_plan*& slot, int64_t n, int64_t C, int64_t W, const icikt_opts& o, icikt_plan** out) {
   icikt_plan* p = slot;
   if (p && p->n == n && p->C == C && p->P == W && p->opts.device == o.device && p->opts.include_diag == o.include_diag) {
-    p->opts.perspective = o.perspective;
-    p->opts.alternative = o.alternative;
-    p->opts.continuity = o.continuity;
-    p->opts.na_inf = o.na_inf;
+    reuse_plan(p, o);
   } else {
     if (p) icikt_plan_destroy(p);
     slot = nullptr;
@@ -2270,95 +2210,7 @@ static int window_plan(icikt_plan*& slot, int64_t n, int64_t C, int64_t W, const
   return ICIKT_OK;
 }
 
-// after a failed call: the cached plan goes, keeping the call's error message
-static void drop_window_plan(icikt_plan*& slot) {
-  const std::string keep = g_err;
-  icikt_plan_destroy(slot);  // waits for whatever the failed call left in flight
-  slot = nullptr;
-  g_err = keep;
-}
-
-static int all_pairs_edges(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                           const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
-                           double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  int rc = check_edge_args(s, n, C, global_na, n_global_na, o, filter, out);
-  if (rc != ICIKT_OK) return rc;
-  rc = select_device(o.device);
-  if (rc != ICIKT_OK) return rc;
-  icikt_edges* res = new (std::nothrow) icikt_edges();
-  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
-  const int64_t ptot = tri_pairs(C) + (o.include_diag ? C : 0);
-  if (ptot == 0) {  // one column, no diagonal: nothing to compute
-    if (max_taumax) *max_taumax = std::nan("");
-    if (timings) std::memset(timings, 0, sizeof(*timings));
-    *out = res;
-    return ICIKT_OK;
-  }
-  const int64_t W = std::min(edge_window(), ptot);
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = nullptr;
-  rc = window_plan(g_cached_edges, n, C, W, o, &p);
-  if (rc == ICIKT_OK) rc = edge_windows(p, s, global_na, n_global_na, *filter, ptot, W, res, max_taumax, timings);
-  if (rc != ICIKT_OK) {
-    drop_window_plan(g_cached_edges);
-    delete res;
-    return rc;
-  }
-  *out = res;
-  return ICIKT_OK;
-}
-
-static int all_pairs_topk(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                          const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max, const TopkOut& out,
-                          double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  int rc = check_topk_args(s, n, C, global_na, n_global_na, o, k, by, out.index);
-  if (rc != ICIKT_OK) return rc;
-  rc = select_device(o.device);
-  if (rc != ICIKT_OK) return rc;
-  const int64_t ptot = tri_pairs(C);
-  if (ptot == 0) {  // one column: no candidate
-    for (int32_t r = 0; r < k; ++r) {
-      out.index[r] = -1;
-      for (double* a : {out.cor, out.raw, out.pvalue, out.taumax, out.completeness})
-        if (a) a[r] = std::nan("");
-    }
-    if (out.n_neighbors) out.n_neighbors[0] = 0;
-    if (max_taumax) *max_taumax = std::nan("");
-    if (timings) std::memset(timings, 0, sizeof(*timings));
-    return ICIKT_OK;
-  }
-  const int64_t W = std::min(edge_window(), ptot);
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = nullptr;
-  rc = window_plan(g_cached_edges, n, C, W, o, &p);
-  if (rc == ICIKT_OK)
-    rc = topk_windows(p, s, global_na, n_global_na, k, by, scale_max != 0, ptot, W, out, max_taumax, timings);
-  if (rc != ICIKT_OK) drop_window_plan(g_cached_edges);
-  return rc;
-}
-
 extern "C" {
-
-int icikt_all_pairs_edges(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                          int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
-                          icikt_edges** out, double* max_taumax, icikt_timings* timings) {
-  return all_pairs_edges(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, filter, out, max_taumax, timings);
-}
-
-int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
-                              int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
-                              const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
-                              icikt_timings* timings) {
-  if (out) *out = nullptr;
-  const int rc = check_csc(colptr, rowidx, values, n, C);
-  if (rc != ICIKT_OK) return rc;
-  return all_pairs_edges(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, filter, out,
-                         max_taumax, timings);
-}
 
 int64_t icikt_edges_count(const icikt_edges* e) { return e ? (int64_t)e->rows.size() : 0; }
 
@@ -2380,25 +2232,6 @@ int icikt_edges_copy(const icikt_edges* e, int32_t* i, int32_t* j, double* cor, 
 }
 
 void icikt_edges_free(icikt_edges* e) { delete e; }
-
-int icikt_all_pairs_topk(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                         int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
-                         int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
-                         double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
-  return all_pairs_topk(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, k, by, scale_max,
-                        TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
-}
-
-int icikt_all_pairs_topk_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
-                             int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
-                             int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
-                             double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
-                             double* max_taumax, icikt_timings* timings) {
-  const int rc = check_csc(colptr, rowidx, values, n, C);
-  if (rc != ICIKT_OK) return rc;
-  return all_pairs_topk(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, k, by, scale_max,
-                        TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
-}
 
 }  // extern "C"
 
@@ -2447,13 +2280,6 @@ static int check_cross_args(const icikt_input* x, const icikt_input* y, int64_t 
     return fail(ICIKT_ERR_BAD_ARG, ranged ? "pair_lo/pair_hi out of [0, Cx * Cy]"
                                           : "this cross call covers all pairs: pair_lo and pair_hi must be 0");
   return ICIKT_OK;
-}
-
-// The cross call's plan (g_cached_edges, windows of W pairs of the Cx + Cy columns of [X | Y]); the caller holds
-// g_cache_mu.
-static int cross_plan(int64_t n, int64_t C, int64_t W, icikt_opts o, icikt_plan** out) {
-  o.pair_lo = o.pair_hi = 0;
-  return window_plan(g_cached_edges, n, C, W, o, out);
 }
 
 // the walk buffers of icikt_cross_pairs and its two result windows (kept with the plan)
@@ -2507,82 +2333,10 @@ static int cross_pair_walk(icikt_plan* p, int64_t Cx, int64_t Cy, int64_t first,
   return walk_windows(p, cross_order(Cx, Cy), first, last, W, tot, select, collect);
 }
 
-// icikt_cross_pairs on one device
-static int cross_pair_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
-                              int32_t n_global_na, int64_t first, int64_t last, int64_t W, double* raw, double* pvalue,
-                              double* taumax, double* completeness, int32_t* status, double* max_taumax,
-                              icikt_timings* timings) {
-  int rc = ensure_cross_buffers(p);
-  if (rc == ICIKT_OK) rc = window_columns(p, sx, global_na, n_global_na, &sy);
-  if (rc != ICIKT_OK) return rc;
-  WalkTotals tot;
-  float d2h_ms = 0.f;
-  rc = cross_pair_walk(p, sx.C, sy.C, first, last, W, raw, pvalue, taumax, completeness, status, tot, d2h_ms);
-  if (rc == ICIKT_OK) rc = finish_walk(p, tot, d2h_ms, timings);
-  if (rc != ICIKT_OK) return rc;
-  if (max_taumax) *max_taumax = max_of_bits(tot.bits);
-  return ICIKT_OK;
-}
-
-static int cross_pairs(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                       int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
-                       double* completeness, int32_t* status, double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  ColumnSource sx, sy;
-  int rc = check_cross_args(x, y, n, global_na, n_global_na, o, true, &sx, &sy);
-  if (rc != ICIKT_OK) return rc;
-  if (!raw) return fail(ICIKT_ERR_BAD_ARG, "raw is NULL");
-  rc = select_device(o.device);
-  if (rc != ICIKT_OK) return rc;
-  const int64_t first = o.pair_lo, last = (o.pair_hi == 0) ? sx.C * sy.C : o.pair_hi;
-  if (last == first) {  // an empty slice: nothing to compute
-    if (max_taumax) *max_taumax = std::nan("");
-    if (timings) std::memset(timings, 0, sizeof(*timings));
-    return ICIKT_OK;
-  }
-  const int64_t W = std::min(edge_window(), last - first);
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = nullptr;
-  rc = cross_plan(n, sx.C + sy.C, W, o, &p);
-  if (rc == ICIKT_OK)
-    rc = cross_pair_windows(p, sx, sy, global_na, n_global_na, first, last, W, raw, pvalue, taumax, completeness, status,
-                            max_taumax, timings);
-  if (rc != ICIKT_OK) drop_window_plan(g_cached_edges);
-  return rc;
-}
-
-static int cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                       int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
-                       double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  ColumnSource sx, sy;
-  int rc = check_filter_args(filter, out);
-  if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
-  if (rc != ICIKT_OK) return rc;
-  rc = select_device(o.device);
-  if (rc != ICIKT_OK) return rc;
-  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
-  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
-  res->j_offset = (int32_t)sx.C;
-  const int64_t ptot = sx.C * sy.C, W = std::min(edge_window(), ptot);
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = nullptr;
-  rc = cross_plan(n, sx.C + sy.C, W, o, &p);
-  if (rc == ICIKT_OK) rc = edge_windows(p, sx, global_na, n_global_na, *filter, ptot, W, res.get(), max_taumax, timings, &sy);
-  if (rc != ICIKT_OK) {
-    drop_window_plan(g_cached_edges);
-    return rc;
-  }
-  *out = res.release();
-  return ICIKT_OK;
-}
-
 // The list rows of a cross top-k call, [c_lo, c_hi) of [X | Y] (X's columns come first, so any choice of sides is one
-// range), and its sides with their raw buffers: x_side rows from 0, y_side rows from Cx - c_lo.
-static int cross_topk_sides(const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, int64_t Cx, int64_t Cy,
-                            int k, int64_t* c_lo, int64_t* c_hi, std::vector<TopkSide>& sides) {
+// range), and its sides: x_side rows from 0, y_side rows from Cx - c_lo.
+static void cross_topk_sides(const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, int64_t Cx, int64_t Cy,
+                             int64_t* c_lo, int64_t* c_hi, std::vector<TopkSide>& sides) {
   *c_lo = x_side ? 0 : Cx;
   *c_hi = y_side ? Cx + Cy : Cx;
   if (x_side) sides.push_back(TopkSide{TopkOut{x_side->index, x_side->n_neighbors, x_side->cor, x_side->raw,
@@ -2591,109 +2345,7 @@ static int cross_topk_sides(const icikt_topk_lists* x_side, const icikt_topk_lis
   if (y_side) sides.push_back(TopkSide{TopkOut{y_side->index, y_side->n_neighbors, y_side->cor, y_side->raw,
                                                y_side->pvalue, y_side->taumax, y_side->completeness},
                                        Cx - *c_lo, Cy, 0, {}, nullptr});
-  for (TopkSide& sd : sides) {
-    const int rc = topk_raw_buffer(sd.out, sd.cols * k, sd.raw_own, &sd.raw);
-    if (rc != ICIKT_OK) return rc;
-  }
-  return ICIKT_OK;
 }
-
-// icikt_cross_topk on one device: lists for the columns of the requested sides only; after the last window each
-// side's rows of the lists go to its caller arrays, and an x-side partner (a column Cx + j of the plan) becomes Y's
-// index j.
-static int cross_topk_windows(icikt_plan* p, const ColumnSource& sx, const ColumnSource& sy, const double* global_na,
-                              int32_t n_global_na, int k, int by, bool scale, int64_t W, const icikt_topk_lists* x_side,
-                              const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings) {
-  const int64_t Cx = sx.C, Cy = sy.C;
-  int64_t c_lo = 0, c_hi = 0;
-  std::vector<TopkSide> sides;
-  int rc = cross_topk_sides(x_side, y_side, Cx, Cy, k, &c_lo, &c_hi, sides);
-  const int64_t L = c_hi - c_lo;
-  if (rc == ICIKT_OK) rc = ensure_topk_buffers(p, W, k, L);
-  if (rc == ICIKT_OK) rc = window_columns(p, sx, global_na, n_global_na, &sy);
-  if (rc != ICIKT_OK) return rc;
-  WalkTotals tot;
-  rc = topk_walk(p, cross_order(Cx, Cy), c_lo, c_hi, k, by, 0, Cx * Cy, W, tot);
-  if (rc != ICIKT_OK) return rc;
-  std::vector<TopkCol> col;
-  try {
-    col.resize((size_t)L);
-  } catch (const std::bad_alloc&) {
-    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
-  }
-  CK(cudaEventRecord(p->ev[6], p->stream));
-  rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)L, p->stream);
-  const int64_t lk = L * k;
-  for (TopkSide& sd : sides) {
-    const int64_t ck = sd.cols * k, at = sd.row0 * k;
-    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index, p->d_tidx + at, sizeof(int32_t) * (size_t)ck, p->stream);
-    double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
-    for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
-      if (host_field[f])
-        rc = staged_copy_out(p, host_field[f], p->d_tlist + f * lk + at, sizeof(double) * (size_t)ck, p->stream);
-  }
-  if (rc != ICIKT_OK) return rc;
-  CK(cudaEventRecord(p->ev[7], p->stream));
-  CK(cudaEventSynchronize(p->ev[7]));
-  const float d2h_ms = ev_ms(p->ev[6], p->ev[7]);
-  const double M = max_of_bits(tot.bits);
-  topk_sides_finish(sides, k, [&](int64_t row) { return col[(size_t)row].n; }, scale, M);
-  rc = finish_walk(p, tot, d2h_ms, timings);
-  if (rc != ICIKT_OK) return rc;
-  if (max_taumax) *max_taumax = M;
-  return ICIKT_OK;
-}
-
-static int cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                      int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
-                      const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
-                      icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  int rc = check_k_by(k, by);
-  if (rc != ICIKT_OK) return rc;
-  if (!x_side && !y_side) return fail(ICIKT_ERR_BAD_ARG, "x_side and y_side are both NULL");
-  if ((x_side && !x_side->index) || (y_side && !y_side->index))
-    return fail(ICIKT_ERR_BAD_ARG, x_side && !x_side->index ? "x_side->index is NULL" : "y_side->index is NULL");
-  ColumnSource sx, sy;
-  rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
-  if (rc != ICIKT_OK) return rc;
-  rc = select_device(o.device);
-  if (rc != ICIKT_OK) return rc;
-  const int64_t W = std::min(edge_window(), sx.C * sy.C);
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = nullptr;
-  rc = cross_plan(n, sx.C + sy.C, W, o, &p);
-  if (rc == ICIKT_OK)
-    rc = cross_topk_windows(p, sx, sy, global_na, n_global_na, k, by, scale_max != 0, W, x_side, y_side, max_taumax,
-                            timings);
-  if (rc != ICIKT_OK) drop_window_plan(g_cached_edges);
-  return rc;
-}
-
-extern "C" {
-
-int icikt_cross_pairs(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                      int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
-                      double* completeness, int32_t* status, double* max_taumax, icikt_timings* timings) {
-  return cross_pairs(x, y, n, global_na, n_global_na, opts, raw, pvalue, taumax, completeness, status, max_taumax,
-                     timings);
-}
-
-int icikt_cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                      int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
-                      double* max_taumax, icikt_timings* timings) {
-  return cross_edges(x, y, n, global_na, n_global_na, opts, filter, out, max_taumax, timings);
-}
-
-int icikt_cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                     int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
-                     const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
-                     icikt_timings* timings) {
-  return cross_topk(x, y, n, global_na, n_global_na, opts, k, by, scale_max, x_side, y_side, max_taumax, timings);
-}
-
-}  // extern "C"
 
 static int pairwise_completeness_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na,
                                       int32_t n_global_na, int32_t device, const int32_t* pi, const int32_t* pj,
@@ -2865,13 +2517,7 @@ int enable_peers(const MultiJob& J, int k) {
 // columns are those of [X | Y]: a shard that straddles column Cx uploads X's part, then Y's (upload_span).
 int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
   const int64_t cnt = J.pair_lo(k + 1) - J.pair_lo(k);
-  if (!J.gather) {
-    if (cnt <= 0 || rc != ICIKT_OK) return rc;
-    if (J.y) return window_columns(p, J.src, J.global_na, J.n_global_na, J.y);
-    rc = J.src.csc() ? upload_columns(p, J.src, 0, J.C) : icikt_plan_upload(p, J.src.data, J.src.ld);
-    if (rc == ICIKT_OK) rc = icikt_plan_columns(p, J.global_na, J.n_global_na);
-    return rc;
-  }
+  if (!J.gather) return cnt <= 0 || rc != ICIKT_OK ? rc : window_columns(p, J.src, J.global_na, J.n_global_na, J.y);
   int x_launches = 0;
   if (rc == ICIKT_OK) rc = upload_span(p, J.src, J.y, J.col_lo(k), J.col_lo(k + 1), &x_launches);
   if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
@@ -2920,10 +2566,7 @@ int multi_worker_pairs(MultiJob& J, int k, icikt_plan** out) {
   icikt_plan* p = nullptr;
   if (cache_matches(slot, J.n, J.C, o, false) && (o.perspective != ICIKT_PERSPECTIVE_COMPLETE || slot->d_pw)) {
     p = slot;
-    p->opts.perspective = o.perspective;
-    p->opts.alternative = o.alternative;
-    p->opts.continuity = o.continuity;
-    p->opts.na_inf = o.na_inf;
+    reuse_plan(p, o);
   } else {
     if (slot) { icikt_plan_destroy(slot); slot = nullptr; }
     rc = icikt_plan_create(&p, J.n, J.C, nullptr, nullptr, 0, &o);
@@ -2962,6 +2605,32 @@ int multi_collect(const std::vector<MultiWork>& work, double* max_taumax, icikt_
   return ICIKT_OK;
 }
 
+// The workers of J: w.rc = body(k, w) for worker k, on the calling thread when there is one worker, on a thread each
+// otherwise.  A worker that fails keeps its message and drops its cached plan slots[k]; then multi_collect.  The
+// caller holds g_cache_mu (the cached plans are not re-entrant).
+template <class Body>
+int run_workers(const MultiJob& J, icikt_plan** slots, std::vector<MultiWork>& work, double* max_taumax,
+                icikt_timings* timings, Body&& body) {
+  work.assign((size_t)J.n_devices, MultiWork{});
+  auto run = [&](int k) {
+    MultiWork& w = work[(size_t)k];
+    w.rc = body(k, w);
+    if (w.rc != ICIKT_OK) {
+      w.err = g_err;  // thread-local message of this worker
+      icikt_plan_destroy(slots[k]);  // waits for whatever the failed worker left in flight
+      slots[k] = nullptr;
+    }
+  };
+  if (J.n_devices == 1) {
+    run(0);
+  } else {
+    std::vector<std::thread> threads;
+    for (int k = 0; k < J.n_devices; ++k) threads.emplace_back(run, k);
+    for (auto& t : threads) t.join();
+  }
+  return multi_collect(work, max_taumax, timings);
+}
+
 int all_pairs_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
                          const icikt_opts* opts, const int32_t* devices, int32_t n_devices, double* raw,
                          double* pvalue, double* taumax, double* completeness, int32_t* status, int64_t* counts,
@@ -2969,6 +2638,7 @@ int all_pairs_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doub
   if ((!s.data && !s.csc()) || !raw) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
   if (n_devices < 1 || n_devices > 64) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..64");
   if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
+  if (!s.csc() && s.ld < n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
   MultiJob J(n_devices);
   J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
   J.devices = devices;
@@ -2977,27 +2647,18 @@ int all_pairs_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doub
   J.ptot = tri_pairs(C) + (J.base.include_diag ? C : 0);
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
   multi_probe_peers(J);
-  std::vector<MultiWork> work((size_t)n_devices);
-  std::vector<std::thread> threads;
-  for (int k = 0; k < n_devices; ++k) {
-    threads.emplace_back([&, k]() {
-      MultiWork& w = work[(size_t)k];
-      icikt_plan* p = nullptr;
-      w.rc = multi_worker_pairs(J, k, &p);
-      const int64_t lo = J.pair_lo(k), cnt = J.pair_lo(k + 1) - lo;
-      if (w.rc == ICIKT_OK && cnt > 0)
-        w.rc = icikt_plan_download(p, raw + lo, pvalue ? pvalue + lo : nullptr, taumax ? taumax + lo : nullptr,
-                                   completeness ? completeness + lo : nullptr, status ? status + lo : nullptr,
-                                   counts ? counts + lo * ICIKT_NCOUNTS : nullptr, &w.mx);
-      if (w.rc == ICIKT_OK && cnt > 0) w.rc = icikt_plan_timings(p, &w.tm);
-      if (w.rc != ICIKT_OK) {
-        w.err = g_err;  // thread-local message of this worker
-        if (g_cached_multi[k]) { icikt_plan_destroy(g_cached_multi[k]); g_cached_multi[k] = nullptr; }
-      }
-    });
-  }
-  for (auto& t : threads) t.join();
-  return multi_collect(work, max_taumax, timings);
+  std::vector<MultiWork> work;
+  return run_workers(J, g_cached_multi, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
+    icikt_plan* p = nullptr;
+    int rc = multi_worker_pairs(J, k, &p);
+    const int64_t lo = J.pair_lo(k), cnt = J.pair_lo(k + 1) - lo;
+    if (rc == ICIKT_OK && cnt > 0)
+      rc = icikt_plan_download(p, raw + lo, pvalue ? pvalue + lo : nullptr, taumax ? taumax + lo : nullptr,
+                               completeness ? completeness + lo : nullptr, status ? status + lo : nullptr,
+                               counts ? counts + lo * ICIKT_NCOUNTS : nullptr, &w.mx);
+    if (rc == ICIKT_OK && cnt > 0) rc = icikt_plan_timings(p, &w.tm);
+    return rc;
+  });
 }
 
 int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
@@ -3026,103 +2687,95 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
     return matrices_impl(s, n, C, global_na, n_global_na, nullptr, nullptr, 0, &base, scale_max, diag_good, n_good,
                          cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
   }
+  if (!s.csc() && s.ld < n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
   double* outs[5] = {cor, raw, pvalue, taumax, completeness};
-  std::vector<MultiWork> work((size_t)n_devices);
+  std::vector<MultiWork> work;
   std::vector<int32_t> good((size_t)C, 0);
   if (n_good) std::copy(n_good, n_good + C, good.begin());
   std::vector<icikt_plan*> plans((size_t)n_devices, nullptr);
-  std::vector<std::thread> threads;
-  for (int k = 0; k < n_devices; ++k) {
-    threads.emplace_back([&, k]() {
-      MultiWork& w = work[(size_t)k];
-      icikt_plan* p = nullptr;
-      w.rc = multi_worker_pairs(J, k, &p);
-      unsigned long long bits = 0;
-      if (w.rc == ICIKT_OK) {
-        if (cudaMemcpyAsync(&bits, p->d_maxbits, sizeof(bits), cudaMemcpyDeviceToHost, p->stream) != cudaSuccess ||
-            cudaStreamSynchronize(p->stream) != cudaSuccess)
-          w.rc = cuda_fail(cudaGetLastError(), "pair kernel");
+  const int rc = run_workers(J, g_cached_multi, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
+    icikt_plan* p = nullptr;
+    w.rc = multi_worker_pairs(J, k, &p);
+    unsigned long long bits = 0;
+    if (w.rc == ICIKT_OK) {
+      if (cudaMemcpyAsync(&bits, p->d_maxbits, sizeof(bits), cudaMemcpyDeviceToHost, p->stream) != cudaSuccess ||
+          cudaStreamSynchronize(p->stream) != cudaSuccess)
+        w.rc = cuda_fail(cudaGetLastError(), "pair kernel");
+    }
+    if (w.rc == ICIKT_OK && bits) std::memcpy(&w.mx, &bits, sizeof(bits));
+    if (w.rc == ICIKT_OK && k == 0 && diag_good && !n_good) {  // n_good = n - missing rows (R/kendalltau.R:165)
+      w.rc = icikt_plan_column_info(p, good.data());
+      for (int64_t c = 0; c < C && w.rc == ICIKT_OK; ++c) good[(size_t)c] = (int32_t)n - good[(size_t)c];
+    }
+    plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
+    J.barrier.wait();  // every slice of the pair results is complete on its device
+    bool all_ok = true;
+    double mx = std::nan("");
+    for (int j = 0; j < n_devices; ++j) {
+      all_ok = all_ok && plans[(size_t)j] != nullptr;
+      if (work[(size_t)j].mx == work[(size_t)j].mx && !(mx >= work[(size_t)j].mx)) mx = work[(size_t)j].mx;
+    }
+    if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to compute its pairs");
+    if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
+    if (w.rc == ICIKT_OK) w.rc = [&]() -> int {
+      const int64_t c_lo = J.col_lo(k), c_hi = J.col_lo(k + 1);
+      const size_t blk = (size_t)C * (size_t)(c_hi - c_lo);
+      CK(cudaSetDevice(p->device));
+      if (p->mat_elems < 5 * blk) {
+        cudaFree(p->d_mat);
+        p->d_mat = nullptr;
+        p->mat_elems = 0;
+        if (dmalloc(&p->d_mat, 5 * blk) != cudaSuccess) {
+          cudaGetLastError();
+          return fail(ICIKT_ERR_ALLOC, "device allocation of the result matrix block failed");
+        }
+        p->mat_elems = 5 * blk;
       }
-      if (w.rc == ICIKT_OK && bits) std::memcpy(&w.mx, &bits, sizeof(bits));
-      if (w.rc == ICIKT_OK && k == 0 && diag_good && !n_good) {  // n_good = n - missing rows (R/kendalltau.R:165)
-        w.rc = icikt_plan_column_info(p, good.data());
-        for (int64_t c = 0; c < C && w.rc == ICIKT_OK; ++c) good[(size_t)c] = (int32_t)n - good[(size_t)c];
+      if (!p->d_hist) CK(dmalloc(&p->d_hist, 16));
+      if (!p->d_ngood) CK(dmalloc(&p->d_ngood, (size_t)C));
+      {
+        const int r3 = ensure_stage(p);
+        if (r3 != ICIKT_OK) return r3;
       }
-      plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
-      J.barrier.wait();  // every slice of the pair results is complete on its device
-      bool all_ok = true;
-      double mx = std::nan("");
+      CK(cudaEventRecord(p->ev[6], p->stream));
+      CK(cudaMemsetAsync(p->d_hist, 0, 16 * sizeof(unsigned long long), p->stream));
+      BlockFill f{};
+      f.n_dev = n_devices;
       for (int j = 0; j < n_devices; ++j) {
-        all_ok = all_ok && plans[(size_t)j] != nullptr;
-        if (work[(size_t)j].mx == work[(size_t)j].mx && !(mx >= work[(size_t)j].mx)) mx = work[(size_t)j].mx;
+        const icikt_plan* q = plans[(size_t)j];
+        f.tau[j] = q->d_tau; f.pvalue[j] = q->d_p; f.taumax[j] = q->d_tm; f.completeness[j] = q->d_comp;
+        f.status[j] = q->d_status;
+        f.pair_lo[j] = J.pair_lo(j);
       }
-      if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to compute its pairs");
-      if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
-      if (w.rc == ICIKT_OK) w.rc = [&]() -> int {
-        const int64_t c_lo = J.col_lo(k), c_hi = J.col_lo(k + 1);
-        const size_t blk = (size_t)C * (size_t)(c_hi - c_lo);
-        CK(cudaSetDevice(p->device));
-        if (p->mat_elems < 5 * blk) {
-          cudaFree(p->d_mat);
-          p->d_mat = nullptr;
-          p->mat_elems = 0;
-          if (dmalloc(&p->d_mat, 5 * blk) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(ICIKT_ERR_ALLOC, "device allocation of the result matrix block failed");
-          }
-          p->mat_elems = 5 * blk;
-        }
-        if (!p->d_hist) CK(dmalloc(&p->d_hist, 16));
-        if (!p->d_ngood) CK(dmalloc(&p->d_ngood, (size_t)C));
-        {
-          const int r3 = ensure_stage(p);
-          if (r3 != ICIKT_OK) return r3;
-        }
-        CK(cudaEventRecord(p->ev[6], p->stream));
-        CK(cudaMemsetAsync(p->d_hist, 0, 16 * sizeof(unsigned long long), p->stream));
-        BlockFill f{};
-        f.n_dev = n_devices;
-        for (int j = 0; j < n_devices; ++j) {
-          const icikt_plan* q = plans[(size_t)j];
-          f.tau[j] = q->d_tau; f.pvalue[j] = q->d_p; f.taumax[j] = q->d_tm; f.completeness[j] = q->d_comp;
-          f.status[j] = q->d_status;
-          f.pair_lo[j] = J.pair_lo(j);
-        }
-        f.pair_lo[n_devices] = ptot;
-        f.n = n; f.C = C; f.c_lo = c_lo; f.c_hi = c_hi;
-        f.scale_max = scale_max != 0; f.diag_good = diag_good != 0;
-        f.max_taumax = mx;
-        f.n_good = p->d_ngood;
-        int best = 1;
-        if (diag_good) {
-          CK(cudaMemcpyAsync(p->d_ngood, good.data(), sizeof(int32_t) * (size_t)C, cudaMemcpyHostToDevice, p->stream));
-          best = 0;
-          for (int64_t c = 0; c < C; ++c) best = std::max(best, good[(size_t)c]);
-        }
-        f.best_good = best;
-        for (int q = 0; q < 5; ++q) f.m[q] = outs[q] ? p->d_mat + (size_t)q * blk : nullptr;
-        f.hist = p->d_hist;
-        if (launch_matrix_block_fill(f, p->stream) < 0) return launch_fail("matrix block fill kernel");
-        for (int q = 0; q < 5; ++q)
-          if (outs[q] && blk) {
-            const int r2 = staged_copy_out(p, outs[q] + (size_t)c_lo * (size_t)C, f.m[q], sizeof(double) * blk, p->stream);
-            if (r2 != ICIKT_OK) return r2;
-          }
-        CK(cudaMemcpyAsync(w.hist, p->d_hist, sizeof(w.hist), cudaMemcpyDeviceToHost, p->stream));
-        CK(cudaEventRecord(p->ev[7], p->stream));
-        CK(cudaStreamSynchronize(p->stream));
-        return icikt_plan_timings(p, &w.tm);
-      }();
-      J.barrier.wait();  // nobody's results are freed before every block has been filled
-      if (w.rc != ICIKT_OK) {
-        w.err = g_err;
-        if (g_cached_multi[k]) { icikt_plan_destroy(g_cached_multi[k]); g_cached_multi[k] = nullptr; }
+      f.pair_lo[n_devices] = ptot;
+      f.n = n; f.C = C; f.c_lo = c_lo; f.c_hi = c_hi;
+      f.scale_max = scale_max != 0; f.diag_good = diag_good != 0;
+      f.max_taumax = mx;
+      f.n_good = p->d_ngood;
+      int best = 1;
+      if (diag_good) {
+        CK(cudaMemcpyAsync(p->d_ngood, good.data(), sizeof(int32_t) * (size_t)C, cudaMemcpyHostToDevice, p->stream));
+        best = 0;
+        for (int64_t c = 0; c < C; ++c) best = std::max(best, good[(size_t)c]);
       }
-    });
-  }
-  for (auto& t : threads) t.join();
-  const int rc = multi_collect(work, max_taumax, timings);
+      f.best_good = best;
+      for (int q = 0; q < 5; ++q) f.m[q] = outs[q] ? p->d_mat + (size_t)q * blk : nullptr;
+      f.hist = p->d_hist;
+      if (launch_matrix_block_fill(f, p->stream) < 0) return launch_fail("matrix block fill kernel");
+      for (int q = 0; q < 5; ++q)
+        if (outs[q] && blk) {
+          const int r2 = staged_copy_out(p, outs[q] + (size_t)c_lo * (size_t)C, f.m[q], sizeof(double) * blk, p->stream);
+          if (r2 != ICIKT_OK) return r2;
+        }
+      CK(cudaMemcpyAsync(w.hist, p->d_hist, sizeof(w.hist), cudaMemcpyDeviceToHost, p->stream));
+      CK(cudaEventRecord(p->ev[7], p->stream));
+      CK(cudaStreamSynchronize(p->stream));
+      return icikt_plan_timings(p, &w.tm);
+    }();
+    J.barrier.wait();  // nobody's results are freed before every block has been filled
+    return w.rc;
+  });
   if (rc != ICIKT_OK) return rc;
   if (status_counts) {
     int64_t bad = 0;
@@ -3136,22 +2789,33 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
   return ICIKT_OK;
 }
 
-// ---- the filtered calls over several devices: the pair order sliced as in icikt_all_pairs_multi, every slice
-// walked window by window on its device, the per-device results combined exactly
+// ---- the windowed calls (filtered, top-k and cross) on one device or several: the pair order sliced as in
+// icikt_all_pairs_multi, every slice walked window by window on its device, the per-device results combined exactly.
+// A single-device call is the job of one worker, run on the calling thread.
+
+icikt_opts opts_or_default(const icikt_opts* opts) {
+  icikt_opts o;
+  if (opts) o = *opts; else icikt_default_opts(&o);
+  return o;
+}
 
 int check_window_devices(int32_t n_devices) {
   if (n_devices < 1 || n_devices > kMaxMatrixDevices) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..16");
   return ICIKT_OK;
 }
 
-// Worker k of a filtered multi-device call up to its window walk: its window plan (cached per worker slot, windows of
-// min(ICIKT_EDGE_WINDOW, its slice) pairs and at least one) and the column phase.
+// The cached window plans of J's workers: one worker takes the single-device slot, several take one slot each, so
+// that one-device and multi-device calls alternated on the same data do not reallocate each other's plans.
+icikt_plan** window_slots(const MultiJob& J) { return J.n_devices == 1 ? &g_cached_edges : g_cached_wmulti; }
+
+// Worker k of a windowed job up to its window walk: its window plan (windows of min(ICIKT_EDGE_WINDOW, its slice)
+// pairs and at least one) and the column phase.
 int window_multi_worker(MultiJob& J, int k, icikt_plan** out) {
   icikt_opts o = J.base;
   o.device = J.device_of(k);
   const int64_t W = std::max<int64_t>(1, std::min(edge_window(), J.pair_lo(k + 1) - J.pair_lo(k)));
   icikt_plan* p = nullptr;
-  int rc = window_plan(g_cached_wmulti[k], J.n, J.C, W, o, &p);
+  int rc = window_plan(window_slots(J)[k], J.n, J.C, W, o, &p);
   *out = p;
   rc = multi_worker_columns(J, k, p, rc);
   if (rc == ICIKT_OK) CK(cudaSetDevice(p->device));
@@ -3164,88 +2828,108 @@ int with_order(const MultiJob& J, const icikt_plan* p, Walk&& walk) {
   return J.y ? walk(cross_order(J.src.C, J.y->C)) : walk(combn_order(p));
 }
 
+// the result of a job without pairs: no maximum, no time
+int no_pairs(double* max_taumax, icikt_timings* timings) {
+  if (max_taumax) *max_taumax = std::nan("");
+  if (timings) std::memset(timings, 0, sizeof(*timings));
+  return ICIKT_OK;
+}
+
 // The filtered call over the devices of J, its arguments checked: every worker walks its slice against the shared
-// EdgeHeld, then the rows are joined in worker order (the slices are contiguous and in order, so are the rows) and
-// edge_result trims them with the final maximum.
-int edges_multi_run(MultiJob& J, const icikt_edge_filter& f, icikt_edges* res, double* max_taumax,
-                    icikt_timings* timings) {
-  const int n_devices = J.n_devices;
-  std::vector<MultiWork> work((size_t)n_devices);
-  std::vector<std::vector<EdgeRow>> rows((size_t)n_devices);
-  std::vector<unsigned long long> bits((size_t)n_devices, 0);
+// EdgeHeld, then the rows are joined in worker order (the slices are contiguous and in order, so are the rows; the
+// first worker's rows are moved, not copied) and edge_result trims them with the final maximum.
+int edges_run(MultiJob& J, const icikt_edge_filter& f, icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  int rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
+  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
+  res->j_offset = J.y ? (int32_t)J.src.C : 0;
+  if (J.ptot == 0) {  // one column, no diagonal: nothing to compute
+    *out = res.release();
+    return no_pairs(max_taumax, timings);
+  }
+  std::vector<MultiWork> work;
+  std::vector<std::vector<EdgeRow>> rows((size_t)J.n_devices);
+  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
   EdgeHeld held;
   {
     std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
     multi_probe_peers(J);
-    std::vector<std::thread> threads;
-    for (int k = 0; k < n_devices; ++k) {
-      threads.emplace_back([&, k]() {
-        MultiWork& w = work[(size_t)k];
-        icikt_plan* p = nullptr;
-        w.rc = window_multi_worker(J, k, &p);
-        const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
-        if (w.rc == ICIKT_OK && hi > lo) {
-          WalkTotals tot;
-          float d2h_ms = 0.f;
-          w.rc = ensure_edge_buffers(p, p->P);
-          if (w.rc == ICIKT_OK)
-            w.rc = with_order(J, p, [&](const auto& order) {
-              return edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
-            });
-          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
-          bits[(size_t)k] = tot.bits;
-        }
-        if (w.rc != ICIKT_OK) {
-          w.err = g_err;  // thread-local message of this worker
-          drop_window_plan(g_cached_wmulti[k]);
-        }
-      });
-    }
-    for (auto& t : threads) t.join();
+    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
+      icikt_plan* p = nullptr;
+      int r = window_multi_worker(J, k, &p);
+      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
+      if (r != ICIKT_OK || hi <= lo) return r;
+      WalkTotals tot;
+      float d2h_ms = 0.f;
+      r = ensure_edge_buffers(p, p->P);
+      if (r == ICIKT_OK)
+        r = with_order(J, p, [&](const auto& order) {
+          return edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
+        });
+      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
+      bits[(size_t)k] = tot.bits;
+      return r;
+    });
   }
-  int rc = multi_collect(work, nullptr, timings);
   if (rc != ICIKT_OK) return rc;
   size_t total = 0;
   for (const auto& r : rows) total += r.size();
+  res->rows = std::move(rows[0]);
   try {
     res->rows.reserve(total);
   } catch (const std::bad_alloc&) {
     return fail(ICIKT_ERR_ALLOC, "out of host memory for the selected rows");
   }
-  for (auto& r : rows) {
-    res->rows.insert(res->rows.end(), r.begin(), r.end());
-    std::vector<EdgeRow>().swap(r);
+  for (size_t k = 1; k < rows.size(); ++k) {
+    res->rows.insert(res->rows.end(), rows[k].begin(), rows[k].end());
+    std::vector<EdgeRow>().swap(rows[k]);
   }
   const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
-  rc = edge_result(res, f, M);
+  rc = edge_result(res.get(), f, M);
   if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = M;
+  *out = res.release();
   return ICIKT_OK;
 }
 
-int edges_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                     const icikt_opts* opts, const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
-                     icikt_edges** out, double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
+int edges_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+               const icikt_opts& o, const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
+               icikt_edges** out, double* max_taumax, icikt_timings* timings) {
   int rc = check_edge_args(s, n, C, global_na, n_global_na, o, filter, out);
   if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
   if (rc != ICIKT_OK) return rc;
-  const int64_t ptot = tri_pairs(C) + (o.include_diag ? C : 0);
   MultiJob J(n_devices);
   J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.ptot = ptot;
-  if (n_devices == 1 || ptot == 0) {
-    o.device = J.device_of(0);
-    return all_pairs_edges(s, n, C, global_na, n_global_na, &o, filter, out, max_taumax, timings);
+  J.devices = devices; J.base = o; J.ptot = tri_pairs(C) + (o.include_diag ? C : 0);
+  return edges_run(J, *filter, out, max_taumax, timings);
+}
+
+// The one-worker counterpart of topk_merge_block: the worker's lists are the result, copied straight from its plan
+// into the arrays of every side; held[r] receives row r's entries, d2h_ms the time of the copy.
+int topk_copy_lists(icikt_plan* p, int64_t L, int K, const std::vector<TopkSide>& sides, int32_t* held, float* d2h_ms) {
+  std::vector<TopkCol> col;
+  try {
+    col.resize((size_t)L);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
   }
-  rc = select_device(J.device_of(0));
+  CK(cudaEventRecord(p->ev[6], p->stream));
+  int rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)L, p->stream);
+  const int64_t lk = L * K;
+  for (const TopkSide& sd : sides) {
+    const int64_t ck = sd.cols * K, at = sd.row0 * K;
+    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index, p->d_tidx + at, sizeof(int32_t) * (size_t)ck, p->stream);
+    double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
+    for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
+      if (host_field[f])
+        rc = staged_copy_out(p, host_field[f], p->d_tlist + f * lk + at, sizeof(double) * (size_t)ck, p->stream);
+  }
   if (rc != ICIKT_OK) return rc;
-  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
-  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
-  rc = edges_multi_run(J, *filter, res.get(), max_taumax, timings);
-  if (rc != ICIKT_OK) return rc;
-  *out = res.release();
+  CK(cudaEventRecord(p->ev[7], p->stream));
+  CK(cudaEventSynchronize(p->ev[7]));
+  *d2h_ms = ev_ms(p->ev[6], p->ev[7]);
+  for (int64_t r = 0; r < L; ++r) held[r] = col[(size_t)r].n;
   return ICIKT_OK;
 }
 
@@ -3300,12 +2984,20 @@ int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<
   return ICIKT_OK;
 }
 
-// The top-k call over the devices of J, its arguments checked and peer access found: every worker keeps the lists of
-// rows [c_lo, c_hi) (columns of the plan) for its slice; after a barrier, worker k merges its block of rows into
-// the sides' arrays; then the host shifts the partners and pads (topk_sides_finish).
-int topk_multi_run(MultiJob& J, int K, int by, bool scale, int64_t c_lo, int64_t c_hi, std::vector<TopkSide>& sides,
-                   double* max_taumax, icikt_timings* timings) {
-  const int n_devices = J.n_devices;
+// The top-k call over the devices of J, its arguments checked: every worker keeps the lists of rows [c_lo, c_hi)
+// (columns of the plan) for its slice.  One worker copies its lists out (topk_copy_lists); several merge a block of
+// rows each into the sides' arrays after a barrier (topk_merge_block).  Then the host shifts the partners and pads
+// (topk_sides_finish).
+int topk_run(MultiJob& J, int K, int by, bool scale, int64_t c_lo, int64_t c_hi, std::vector<TopkSide>& sides,
+             double* max_taumax, icikt_timings* timings) {
+  int rc = select_device(J.device_of(0));
+  for (TopkSide& sd : sides)
+    if (rc == ICIKT_OK) rc = topk_raw_buffer(sd.out, sd.cols * K, sd.raw_own, &sd.raw);
+  if (rc != ICIKT_OK) return rc;
+  if (J.ptot == 0) {  // one column: no candidate, its list is padding
+    topk_sides_finish(sides, K, [](int64_t) { return 0; }, scale, std::nan(""));
+    return no_pairs(max_taumax, timings);
+  }
   const int64_t L = c_hi - c_lo;
   std::vector<int32_t> held;
   try {
@@ -3313,44 +3005,41 @@ int topk_multi_run(MultiJob& J, int K, int by, bool scale, int64_t c_lo, int64_t
   } catch (const std::bad_alloc&) {
     return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
   }
-  std::vector<MultiWork> work((size_t)n_devices);
-  std::vector<unsigned long long> bits((size_t)n_devices, 0);
-  std::vector<icikt_plan*> plans((size_t)n_devices, nullptr);
+  std::vector<MultiWork> work;
+  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
+  std::vector<icikt_plan*> plans((size_t)J.n_devices, nullptr);
   {
     std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
-    std::vector<std::thread> threads;
-    for (int k = 0; k < n_devices; ++k) {
-      threads.emplace_back([&, k]() {
-        MultiWork& w = work[(size_t)k];
-        icikt_plan* p = nullptr;
-        w.rc = window_multi_worker(J, k, &p);
-        if (w.rc == ICIKT_OK) {
-          WalkTotals tot;
-          w.rc = ensure_topk_buffers(p, p->P, K, L);
-          if (w.rc == ICIKT_OK)
-            w.rc = with_order(J, p, [&](const auto& order) {
-              return topk_walk(p, order, c_lo, c_hi, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
-            });
-          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, 0.f, &w.tm);
-          bits[(size_t)k] = tot.bits;
-        }
-        plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
-        J.barrier.wait();  // every device's lists are complete
-        bool all_ok = true;
-        for (int j = 0; j < n_devices; ++j) all_ok = all_ok && plans[(size_t)j] != nullptr;
-        if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to select its lists");
-        if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
-        if (w.rc == ICIKT_OK) w.rc = topk_merge_block(J, k, p, plans, L, K, by, sides, held.data(), w.tm);
-        J.barrier.wait();  // nobody's lists are freed (or reused) before every block has been merged
-        if (w.rc != ICIKT_OK) {
-          w.err = g_err;
-          drop_window_plan(g_cached_wmulti[k]);
-        }
-      });
-    }
-    for (auto& t : threads) t.join();
+    multi_probe_peers(J);
+    // devices that cannot read each other's lists: one worker on devices[0] (no gather, no barrier)
+    if (!J.peers_ok) J.n_devices = 1;
+    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
+      icikt_plan* p = nullptr;
+      int r = window_multi_worker(J, k, &p);
+      WalkTotals tot;
+      if (r == ICIKT_OK) r = ensure_topk_buffers(p, p->P, K, L);
+      if (r == ICIKT_OK)
+        r = with_order(J, p, [&](const auto& order) {
+          return topk_walk(p, order, c_lo, c_hi, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
+        });
+      bits[(size_t)k] = tot.bits;
+      if (J.n_devices == 1) {
+        float d2h_ms = 0.f;
+        if (r == ICIKT_OK) r = topk_copy_lists(p, L, K, sides, held.data(), &d2h_ms);
+        return r == ICIKT_OK ? finish_walk(p, tot, d2h_ms, &w.tm) : r;
+      }
+      if (r == ICIKT_OK) r = finish_walk(p, tot, 0.f, &w.tm);
+      plans[(size_t)k] = (r == ICIKT_OK) ? p : nullptr;
+      J.barrier.wait();  // every device's lists are complete
+      bool all_ok = true;
+      for (int j = 0; j < J.n_devices; ++j) all_ok = all_ok && plans[(size_t)j] != nullptr;
+      if (r == ICIKT_OK && !all_ok) r = fail(ICIKT_ERR_CUDA, "a peer device failed to select its lists");
+      if (r == ICIKT_OK) r = enable_peers(J, k);
+      if (r == ICIKT_OK) r = topk_merge_block(J, k, p, plans, L, K, by, sides, held.data(), w.tm);
+      J.barrier.wait();  // nobody's lists are freed (or reused) before every block has been merged
+      return r;
+    });
   }
-  const int rc = multi_collect(work, nullptr, timings);
   if (rc != ICIKT_OK) return rc;
   const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
   topk_sides_finish(sides, K, [&](int64_t row) { return held[(size_t)row]; }, scale, M);
@@ -3358,41 +3047,20 @@ int topk_multi_run(MultiJob& J, int K, int by, bool scale, int64_t c_lo, int64_t
   return ICIKT_OK;
 }
 
-int topk_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                    const icikt_opts* opts, const int32_t* devices, int32_t n_devices, int32_t K, int32_t by,
-                    int32_t scale_max, const TopkOut& out, double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
+int topk_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+              const icikt_opts& o, const int32_t* devices, int32_t n_devices, int32_t K, int32_t by, int32_t scale_max,
+              const TopkOut& out, double* max_taumax, icikt_timings* timings) {
   int rc = check_topk_args(s, n, C, global_na, n_global_na, o, K, by, out.index);
   if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
   if (rc != ICIKT_OK) return rc;
-  const int64_t ptot = tri_pairs(C);
   MultiJob J(n_devices);
   J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.ptot = ptot;
-  rc = select_device(J.device_of(0));
-  if (rc != ICIKT_OK) return rc;
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);
-    multi_probe_peers(J);
-  }
-  if (n_devices == 1 || !J.peers_ok || ptot == 0) {
-    // one device, or devices that cannot read each other's lists: the single-device call
-    o.device = J.device_of(0);
-    return all_pairs_topk(s, n, C, global_na, n_global_na, &o, K, by, scale_max, out, max_taumax, timings);
-  }
-  std::vector<TopkSide> sides(1);
-  sides[0].out = out;
-  sides[0].row0 = 0;
-  sides[0].cols = C;
-  sides[0].shift = 0;
-  rc = topk_raw_buffer(out, C * K, sides[0].raw_own, &sides[0].raw);
-  if (rc != ICIKT_OK) return rc;
-  return topk_multi_run(J, K, by, scale_max != 0, 0, C, sides, max_taumax, timings);
+  J.devices = devices; J.base = o; J.ptot = tri_pairs(C);
+  std::vector<TopkSide> sides{TopkSide{out, 0, C, 0, {}, nullptr}};
+  return topk_run(J, K, by, scale_max != 0, 0, C, sides, max_taumax, timings);
 }
 
-// ---- the cross calls over several devices: the cross order (of the call's range) sliced as above over the
-// Cx + Cy columns of [X | Y]
+// ---- the cross calls: the cross order (of the call's range) sliced as above over the Cx + Cy columns of [X | Y]
 
 // A cross job over pairs [first, last) of the cross order, its arguments checked.  The window plans hold W pairs of
 // a slice: the call's pair range is the job's, not theirs.
@@ -3403,12 +3071,10 @@ void cross_job(MultiJob& J, const ColumnSource& sx, const ColumnSource& sy, int6
   J.first = first; J.ptot = last - first;
 }
 
-int cross_pairs_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                      int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
-                      double* raw, double* pvalue, double* taumax, double* completeness, int32_t* status,
-                      double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
+int cross_pairs_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                     int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices, double* raw,
+                     double* pvalue, double* taumax, double* completeness, int32_t* status, double* max_taumax,
+                     icikt_timings* timings) {
   ColumnSource sx, sy;
   int rc = check_cross_args(x, y, n, global_na, n_global_na, o, true, &sx, &sy);
   if (rc == ICIKT_OK && !raw) rc = fail(ICIKT_ERR_BAD_ARG, "raw is NULL");
@@ -3417,55 +3083,39 @@ int cross_pairs_multi(const icikt_input* x, const icikt_input* y, int64_t n, con
   const int64_t first = o.pair_lo, last = (o.pair_hi == 0) ? sx.C * sy.C : o.pair_hi;
   MultiJob J(n_devices);
   cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, first, last);
-  if (n_devices == 1 || last == first) {
-    o.device = J.device_of(0);
-    return cross_pairs(x, y, n, global_na, n_global_na, &o, raw, pvalue, taumax, completeness, status, max_taumax,
-                       timings);
-  }
   rc = select_device(J.device_of(0));
   if (rc != ICIKT_OK) return rc;
-  std::vector<MultiWork> work((size_t)n_devices);
+  if (J.ptot == 0) return no_pairs(max_taumax, timings);  // an empty slice
+  std::vector<MultiWork> work;
   std::vector<unsigned long long> bits((size_t)n_devices, 0);
   {
     std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
     multi_probe_peers(J);
-    std::vector<std::thread> threads;
-    for (int k = 0; k < n_devices; ++k) {
-      threads.emplace_back([&, k]() {
-        MultiWork& w = work[(size_t)k];
-        icikt_plan* p = nullptr;
-        w.rc = window_multi_worker(J, k, &p);
-        const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1), off = lo - first;
-        if (w.rc == ICIKT_OK && hi > lo) {
-          WalkTotals tot;
-          float d2h_ms = 0.f;
-          w.rc = ensure_cross_buffers(p);
-          if (w.rc == ICIKT_OK)
-            w.rc = cross_pair_walk(p, sx.C, sy.C, lo, hi, p->P, raw + off, pvalue ? pvalue + off : nullptr,
-                                   taumax ? taumax + off : nullptr, completeness ? completeness + off : nullptr,
-                                   status ? status + off : nullptr, tot, d2h_ms);
-          if (w.rc == ICIKT_OK) w.rc = finish_walk(p, tot, d2h_ms, &w.tm);
-          bits[(size_t)k] = tot.bits;
-        }
-        if (w.rc != ICIKT_OK) {
-          w.err = g_err;  // thread-local message of this worker
-          drop_window_plan(g_cached_wmulti[k]);
-        }
-      });
-    }
-    for (auto& t : threads) t.join();
+    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
+      icikt_plan* p = nullptr;
+      int r = window_multi_worker(J, k, &p);
+      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1), off = lo - first;
+      if (r != ICIKT_OK || hi <= lo) return r;
+      WalkTotals tot;
+      float d2h_ms = 0.f;
+      r = ensure_cross_buffers(p);
+      if (r == ICIKT_OK)
+        r = cross_pair_walk(p, sx.C, sy.C, lo, hi, p->P, raw + off, pvalue ? pvalue + off : nullptr,
+                            taumax ? taumax + off : nullptr, completeness ? completeness + off : nullptr,
+                            status ? status + off : nullptr, tot, d2h_ms);
+      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
+      bits[(size_t)k] = tot.bits;
+      return r;
+    });
   }
-  rc = multi_collect(work, nullptr, timings);
   if (rc != ICIKT_OK) return rc;
   if (max_taumax) *max_taumax = max_of_bits(*std::max_element(bits.begin(), bits.end()));
   return ICIKT_OK;
 }
 
-int cross_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                      int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
-                      const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
+int cross_edges_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                     int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices,
+                     const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax, icikt_timings* timings) {
   ColumnSource sx, sy;
   int rc = check_filter_args(filter, out);
   if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
@@ -3473,27 +3123,13 @@ int cross_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, con
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
   cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
-  if (n_devices == 1) {
-    o.device = J.device_of(0);
-    return cross_edges(x, y, n, global_na, n_global_na, &o, filter, out, max_taumax, timings);
-  }
-  rc = select_device(J.device_of(0));
-  if (rc != ICIKT_OK) return rc;
-  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
-  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
-  res->j_offset = (int32_t)sx.C;
-  rc = edges_multi_run(J, *filter, res.get(), max_taumax, timings);
-  if (rc != ICIKT_OK) return rc;
-  *out = res.release();
-  return ICIKT_OK;
+  return edges_run(J, *filter, out, max_taumax, timings);
 }
 
-int cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
-                     int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices, int32_t K,
-                     int32_t by, int32_t scale_max, const icikt_topk_lists* x_side, const icikt_topk_lists* y_side,
-                     double* max_taumax, icikt_timings* timings) {
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
+int cross_topk_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                    int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices, int32_t K,
+                    int32_t by, int32_t scale_max, const icikt_topk_lists* x_side, const icikt_topk_lists* y_side,
+                    double* max_taumax, icikt_timings* timings) {
   int rc = check_k_by(K, by);
   if (rc != ICIKT_OK) return rc;
   if (!x_side && !y_side) return fail(ICIKT_ERR_BAD_ARG, "x_side and y_side are both NULL");
@@ -3505,22 +3141,10 @@ int cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n, cons
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
   cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
-  rc = select_device(J.device_of(0));
-  if (rc != ICIKT_OK) return rc;
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);
-    multi_probe_peers(J);
-  }
-  if (n_devices == 1 || !J.peers_ok) {
-    // one device, or devices that cannot read each other's lists: the single-device call
-    o.device = J.device_of(0);
-    return cross_topk(x, y, n, global_na, n_global_na, &o, K, by, scale_max, x_side, y_side, max_taumax, timings);
-  }
   int64_t c_lo = 0, c_hi = 0;
   std::vector<TopkSide> sides;
-  rc = cross_topk_sides(x_side, y_side, sx.C, sy.C, K, &c_lo, &c_hi, sides);
-  if (rc != ICIKT_OK) return rc;
-  return topk_multi_run(J, K, by, scale_max != 0, c_lo, c_hi, sides, max_taumax, timings);
+  cross_topk_sides(x_side, y_side, sx.C, sy.C, &c_lo, &c_hi, sides);
+  return topk_run(J, K, by, scale_max != 0, c_lo, c_hi, sides, max_taumax, timings);
 }
 
 }  // namespace
@@ -3570,12 +3194,32 @@ int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const
                              status_counts, max_taumax, timings);
 }
 
+int icikt_all_pairs_edges(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                          int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
+                          icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return edges_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, o, &o.device, 1, filter, out, max_taumax,
+                    timings);
+}
+
+int icikt_all_pairs_edges_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                              int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                              const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
+                              icikt_timings* timings) {
+  if (out) *out = nullptr;
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  const icikt_opts o = opts_or_default(opts);
+  return edges_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, o, &o.device, 1, filter, out,
+                    max_taumax, timings);
+}
+
 int icikt_all_pairs_edges_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
                                 int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
                                 const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
                                 icikt_timings* timings) {
-  return edges_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, filter, out,
-                          max_taumax, timings);
+  return edges_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts_or_default(opts), devices, n_devices,
+                    filter, out, max_taumax, timings);
 }
 
 int icikt_all_pairs_edges_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
@@ -3585,8 +3229,29 @@ int icikt_all_pairs_edges_multi_csc(const int64_t* colptr, const int32_t* rowidx
   if (out) *out = nullptr;
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return edges_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices, n_devices,
-                          filter, out, max_taumax, timings);
+  return edges_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts_or_default(opts), devices,
+                    n_devices, filter, out, max_taumax, timings);
+}
+
+int icikt_all_pairs_topk(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                         int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                         int32_t* index, int32_t* n_neighbors, double* cor, double* raw, double* pvalue,
+                         double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return topk_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, o, &o.device, 1, k, by, scale_max,
+                   TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
+}
+
+int icikt_all_pairs_topk_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
+                             int64_t C, const double* global_na, int32_t n_global_na, const icikt_opts* opts,
+                             int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
+                             double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                             double* max_taumax, icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  const icikt_opts o = opts_or_default(opts);
+  return topk_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, o, &o.device, 1, k, by,
+                   scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax, timings);
 }
 
 int icikt_all_pairs_topk_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
@@ -3594,9 +3259,9 @@ int icikt_all_pairs_topk_multi(const double* data, int64_t n, int64_t C, int64_t
                                int32_t k, int32_t by, int32_t scale_max, int32_t* index, int32_t* n_neighbors,
                                double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
                                double* max_taumax, icikt_timings* timings) {
-  return topk_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, k, by,
-                         scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax,
-                         timings);
+  return topk_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts_or_default(opts), devices, n_devices,
+                   k, by, scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness}, max_taumax,
+                   timings);
 }
 
 int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
@@ -3606,32 +3271,57 @@ int icikt_all_pairs_topk_multi_csc(const int64_t* colptr, const int32_t* rowidx,
                                    double* taumax, double* completeness, double* max_taumax, icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return topk_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices, n_devices, k,
-                         by, scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness},
-                         max_taumax, timings);
+  return topk_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts_or_default(opts), devices,
+                   n_devices, k, by, scale_max, TopkOut{index, n_neighbors, cor, raw, pvalue, taumax, completeness},
+                   max_taumax, timings);
+}
+
+int icikt_cross_pairs(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
+                      double* completeness, int32_t* status, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return cross_pairs_impl(x, y, n, global_na, n_global_na, o, &o.device, 1, raw, pvalue, taumax, completeness, status,
+                          max_taumax, timings);
 }
 
 int icikt_cross_pairs_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
                             int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
                             double* raw, double* pvalue, double* taumax, double* completeness, int32_t* status,
                             double* max_taumax, icikt_timings* timings) {
-  return cross_pairs_multi(x, y, n, global_na, n_global_na, opts, devices, n_devices, raw, pvalue, taumax, completeness,
-                           status, max_taumax, timings);
+  return cross_pairs_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, raw, pvalue,
+                          taumax, completeness, status, max_taumax, timings);
+}
+
+int icikt_cross_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                      int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter, icikt_edges** out,
+                      double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return cross_edges_impl(x, y, n, global_na, n_global_na, o, &o.device, 1, filter, out, max_taumax, timings);
 }
 
 int icikt_cross_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
                             int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
                             const icikt_edge_filter* filter, icikt_edges** out, double* max_taumax,
                             icikt_timings* timings) {
-  return cross_edges_multi(x, y, n, global_na, n_global_na, opts, devices, n_devices, filter, out, max_taumax, timings);
+  return cross_edges_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filter, out,
+                          max_taumax, timings);
+}
+
+int icikt_cross_topk(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                     int32_t n_global_na, const icikt_opts* opts, int32_t k, int32_t by, int32_t scale_max,
+                     const icikt_topk_lists* x_side, const icikt_topk_lists* y_side, double* max_taumax,
+                     icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return cross_topk_impl(x, y, n, global_na, n_global_na, o, &o.device, 1, k, by, scale_max, x_side, y_side,
+                         max_taumax, timings);
 }
 
 int icikt_cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
                            int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
                            int32_t k, int32_t by, int32_t scale_max, const icikt_topk_lists* x_side,
                            const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings) {
-  return cross_topk_multi(x, y, n, global_na, n_global_na, opts, devices, n_devices, k, by, scale_max, x_side, y_side,
-                          max_taumax, timings);
+  return cross_topk_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, k, by, scale_max,
+                         x_side, y_side, max_taumax, timings);
 }
 
 int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
