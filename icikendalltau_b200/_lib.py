@@ -22,6 +22,8 @@ TOPK_MAX = 1024
 KERNEL_TILED, KERNEL_NAIVE = 0, 1
 PERSPECTIVE = {"global": 0, "local": 1, "complete": 2}
 ALTERNATIVE = {"two.sided": 0, "less": 1, "greater": 2}
+# R's p.adjust methods offered (ICIKT_PADJ_*); "fdr" is R's alias of "BH", "hommel" is not offered
+PADJ = {"bonferroni": 1, "holm": 2, "hochberg": 3, "BH": 4, "fdr": 4, "BY": 5}
 
 # every symbol include/icikt_b200.h declares (checked by tests/test_abi_cpu.py)
 EXPORTS = [
@@ -42,6 +44,8 @@ EXPORTS = [
     "icikt_all_pairs_edges_multi", "icikt_all_pairs_edges_multi_csc", "icikt_all_pairs_topk_multi",
     "icikt_all_pairs_topk_multi_csc", "icikt_cross_pairs", "icikt_cross_edges", "icikt_cross_topk",
     "icikt_cross_pairs_multi", "icikt_cross_edges_multi", "icikt_cross_topk_multi",
+    "icikt_p_adjust", "icikt_all_pairs_edges_padj", "icikt_all_pairs_edges_padj_multi", "icikt_cross_edges_padj",
+    "icikt_cross_edges_padj_multi", "icikt_edges_copy_padj", "icikt_edges_n_tests",
 ]
 NSTATUS = 10
 
@@ -75,6 +79,10 @@ class Timings(ctypes.Structure):
 class EdgeFilter(ctypes.Structure):
     _fields_ = [("min_abs_cor", ctypes.c_double), ("max_pvalue", ctypes.c_double),
                 ("scale_max", ctypes.c_int32), ("reserved", ctypes.c_int32), ("max_edges", ctypes.c_int64)]
+
+
+class PadjFilter(ctypes.Structure):
+    _fields_ = [("method", ctypes.c_int32), ("reserved", ctypes.c_int32), ("max_padj", ctypes.c_double)]
 
 
 class Input(ctypes.Structure):
@@ -214,6 +222,19 @@ def load():
         f = getattr(L, name + "_multi")
         f.argtypes = a[:6] + [_ip, ctypes.c_int32] + a[6:]
         f.restype = ctypes.c_int
+    # the _padj twins of the edges calls: the matrix as an icikt_input, the icikt_padj_filter after the edge filter
+    ef = [ctypes.POINTER(EdgeFilter), ctypes.POINTER(PadjFilter), ctypes.POINTER(vp), _dp, ctypes.POINTER(Timings)]
+    one = [ctypes.POINTER(Input), ctypes.c_int64, _dp, ctypes.c_int32, ctypes.POINTER(Opts)]
+    for name, lead in (("icikt_all_pairs_edges_padj", one), ("icikt_cross_edges_padj", cross)):
+        getattr(L, name).argtypes = lead + ef
+        getattr(L, name + "_multi").argtypes = lead + [_ip, ctypes.c_int32] + ef
+        getattr(L, name).restype = getattr(L, name + "_multi").restype = ctypes.c_int
+    L.icikt_p_adjust.argtypes = [_dp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, _dp, ctypes.POINTER(ctypes.c_int64)]
+    L.icikt_p_adjust.restype = ctypes.c_int
+    L.icikt_edges_copy_padj.argtypes = [vp, _dp]
+    L.icikt_edges_copy_padj.restype = ctypes.c_int
+    L.icikt_edges_n_tests.argtypes = [vp]
+    L.icikt_edges_n_tests.restype = ctypes.c_int64
     L.icikt_plan_column_info.argtypes = [vp, _ip]
     L.icikt_plan_column_info.restype = ctypes.c_int
     L.icikt_plan_stream.argtypes = [vp]
@@ -394,8 +415,64 @@ def _devices_args(devices):
     return "_multi", (_ptr(dev, _ip), int(dev.size)), dev
 
 
+def padj_method(p_adjust):
+    """ICIKT_PADJ_* of one of R's p.adjust method names; ValueError for "hommel" and unknown names"""
+    if p_adjust not in PADJ:
+        raise ValueError(f"`p_adjust` must be one of {sorted(PADJ)} (hommel is not offered), got {p_adjust!r}")
+    return PADJ[p_adjust]
+
+
+def p_adjust(p, method, device=0):
+    """R's p.adjust(p, method) on the device (icikt_p_adjust), bit for bit: NaN entries are not part of the family
+    and stay NaN, and fewer than two non-NaN values leave p unchanged.  method: "bonferroni", "holm", "hochberg",
+    "BH" (alias "fdr") or "BY".  Returns a float64 array of p's shape."""
+    code = padj_method(method)
+    L = load()
+    a = np.ascontiguousarray(p, dtype=np.float64)
+    out = np.empty_like(a)
+    nt = ctypes.c_int64(0)
+    check(L.icikt_p_adjust(_ptr(a), a.size, code, int(device), _ptr(out), ctypes.byref(nt)))
+    return out
+
+
+def _padj_args(p_adjust, max_padj):
+    """the icikt_padj_filter of run_edges / run_cross_edges, or None without p_adjust"""
+    if p_adjust is None:
+        if max_padj is not None:
+            raise ValueError("`max_padj` bounds the adjusted p-value: give `p_adjust` too")
+        return None
+    return PadjFilter(padj_method(p_adjust), 0, _bound(max_padj))
+
+
+def _input(a):
+    """(icikt_input of one matrix, n, C, the object that owns the memory it points into)"""
+    if is_sparse(a):
+        m = CSC(a)
+        return Input(m.shape[1], None, 0, _ptr(m.colptr), _ptr(m.rowidx), _ptr(m.values)), m.shape[0], m.shape[1], m
+    m = np.asfortranarray(a, dtype=np.float64)
+    if m.ndim != 2:
+        raise ValueError("x and y must be 2-D arrays (features x samples)")
+    return Input(m.shape[1], _ptr(m), m.shape[0], None, None, None), m.shape[0], m.shape[1], m
+
+
+def _edges_out(L, h, adjusted):
+    """the rows of an icikt_edges result as a dict of arrays (with padj and n_tests from a _padj call); frees h"""
+    try:
+        m = int(L.icikt_edges_count(h))
+        out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
+        out.update((k, np.empty(m, dtype=np.float64)) for k in EDGE_NAMES)
+        check(L.icikt_edges_copy(h, _ptr(out["i"]), _ptr(out["j"]), *(_ptr(out[k]) for k in EDGE_NAMES)))
+        if adjusted:
+            out["padj"] = np.empty(m, dtype=np.float64)
+            check(L.icikt_edges_copy_padj(h, _ptr(out["padj"])))
+            out["n_tests"] = int(L.icikt_edges_n_tests(h))
+    finally:
+        L.icikt_edges_free(h)
+    return out
+
+
 def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, devices=None,
-              **opt_kw):
+              p_adjust=None, max_padj=None, **opt_kw):
     """icikt_all_pairs_edges: all pairs, filtered on the device, as a long table of the pairs that pass.
 
     A pair is kept iff it is not degenerate, abs(cor) >= min_abs_cor and pvalue <= max_pvalue (a bound of None is
@@ -404,10 +481,14 @@ def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=T
     (-> icikt_all_pairs_edges_csc).  max_edges > 0 raises IciktError(ERR_LIMIT) when more pairs pass.
     devices: list of CUDA ordinals -> icikt_all_pairs_edges_multi(_csc): every device walks a contiguous slice of the
     pair order; the result is bit for bit the single-device one.
+    p_adjust: one of R's p.adjust methods ("bonferroni", "holm", "hochberg", "BH" or "fdr", "BY") ->
+    icikt_all_pairs_edges_padj(_multi): rows also get padj, bit for bit p.adjust(p_all, p_adjust) over the non-NaN
+    p-values of every pair (p_all: run_pairs' pvalue), and the dict gets n_tests (their number); max_padj keeps the
+    rows with padj <= max_padj (None: no condition) and needs p_adjust.
     Returns a dict of NumPy arrays i, j (int32), cor, raw, pvalue, taumax, completeness, plus max_taumax and
     timings."""
+    adj = _padj_args(p_adjust, max_padj)
     L = load()
-    lead, sfx, n, C, keep_alive = _matrix_args(data)
     msfx, dargs, dev = _devices_args(devices)
     o = make_opts(**opt_kw)
     f = EdgeFilter(_bound(min_abs_cor), _bound(max_pvalue), int(bool(scale_max)), 0, int(max_edges))
@@ -415,15 +496,16 @@ def run_edges(data, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=T
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(getattr(L, "icikt_all_pairs_edges" + msfx + sfx)(*lead, gp, ng, ctypes.byref(o), *dargs, ctypes.byref(f),
-                                                           ctypes.byref(h), ctypes.byref(mx), ctypes.byref(t)))
-    try:
-        m = int(L.icikt_edges_count(h))
-        out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
-        out.update((k, np.empty(m, dtype=np.float64)) for k in EDGE_NAMES)
-        check(L.icikt_edges_copy(h, _ptr(out["i"]), _ptr(out["j"]), *(_ptr(out[k]) for k in EDGE_NAMES)))
-    finally:
-        L.icikt_edges_free(h)
+    if adj is None:
+        lead, sfx, n, C, keep_alive = _matrix_args(data)
+        check(getattr(L, "icikt_all_pairs_edges" + msfx + sfx)(*lead, gp, ng, ctypes.byref(o), *dargs, ctypes.byref(f),
+                                                               ctypes.byref(h), ctypes.byref(mx), ctypes.byref(t)))
+    else:
+        xi, n, C, keep_alive = _input(data)
+        check(getattr(L, "icikt_all_pairs_edges_padj" + msfx)(ctypes.byref(xi), n, gp, ng, ctypes.byref(o), *dargs,
+                                                              ctypes.byref(f), ctypes.byref(adj), ctypes.byref(h),
+                                                              ctypes.byref(mx), ctypes.byref(t)))
+    out = _edges_out(L, h, adj is not None)
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 
@@ -468,17 +550,9 @@ def _cross_inputs(x, y):
     and y may each be a NumPy array or a scipy.sparse matrix"""
     ins, keep = [], []
     for a in (x, y):
-        if is_sparse(a):
-            m = CSC(a)
-            ins.append(Input(m.shape[1], None, 0, _ptr(m.colptr), _ptr(m.rowidx), _ptr(m.values)))
-            shape = m.shape
-        else:
-            m = np.asfortranarray(a, dtype=np.float64)
-            if m.ndim != 2:
-                raise ValueError("x and y must be 2-D arrays (features x samples)")
-            ins.append(Input(m.shape[1], _ptr(m), m.shape[0], None, None, None))
-            shape = m.shape
-        keep.append((m, shape))
+        i, n, c, m = _input(a)
+        ins.append(i)
+        keep.append((m, (n, c)))
     (_, (nx, cx)), (_, (ny, cy)) = keep
     if nx != ny:
         raise ValueError(f"x has {nx} rows and y has {ny}: the cross calls need the same rows")
@@ -512,10 +586,12 @@ def run_cross(x, y, global_na=(), devices=None, **opt_kw):
 
 
 def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale_max=True, max_edges=0, devices=None,
-                    **opt_kw):
+                    p_adjust=None, max_padj=None, **opt_kw):
     """icikt_cross_edges: the pairs of x's columns with y's columns that pass the filter of run_edges, in cross
     order, filtered on the device.  devices: list of CUDA ordinals -> icikt_cross_edges_multi, bit for bit the
-    single-device result.  Returns the dict of run_edges; i indexes x's columns, j y's."""
+    single-device result.  p_adjust / max_padj as in run_edges (-> icikt_cross_edges_padj(_multi)), the family being
+    every pair of the cross order.  Returns the dict of run_edges; i indexes x's columns, j y's."""
+    adj = _padj_args(p_adjust, max_padj)
     L = load()
     xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
     msfx, dargs, dev = _devices_args(devices)
@@ -525,16 +601,15 @@ def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
-    check(getattr(L, "icikt_cross_edges" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
-                                                 *dargs, ctypes.byref(f), ctypes.byref(h), ctypes.byref(mx),
-                                                 ctypes.byref(t)))
-    try:
-        m = int(L.icikt_edges_count(h))
-        out = dict(i=np.empty(m, dtype=np.int32), j=np.empty(m, dtype=np.int32))
-        out.update((k, np.empty(m, dtype=np.float64)) for k in EDGE_NAMES)
-        check(L.icikt_edges_copy(h, _ptr(out["i"]), _ptr(out["j"]), *(_ptr(out[k]) for k in EDGE_NAMES)))
-    finally:
-        L.icikt_edges_free(h)
+    if adj is None:
+        check(getattr(L, "icikt_cross_edges" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
+                                                     *dargs, ctypes.byref(f), ctypes.byref(h), ctypes.byref(mx),
+                                                     ctypes.byref(t)))
+    else:
+        check(getattr(L, "icikt_cross_edges_padj" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng,
+                                                          ctypes.byref(o), *dargs, ctypes.byref(f), ctypes.byref(adj),
+                                                          ctypes.byref(h), ctypes.byref(mx), ctypes.byref(t)))
+    out = _edges_out(L, h, adj is not None)
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
 

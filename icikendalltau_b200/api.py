@@ -223,6 +223,18 @@ def _edge_mask(cor, pvalue, min_abs_cor, max_pvalue):
     return sel
 
 
+def _padj_checks(p_adjust, max_padj, return_matrix):
+    """the argument checks of p_adjust / max_padj; True when the long table gets a padj column"""
+    if p_adjust is None:
+        if max_padj is not None:
+            raise ValueError("`max_padj` bounds the adjusted p-value: give `p_adjust` too")
+        return False
+    _lib.padj_method(p_adjust)
+    if return_matrix:
+        raise ValueError("`p_adjust` and `max_padj` add a column to the long table: pass return_matrix=False")
+    return True
+
+
 def _reshape(names, pi, pj, cols):
     C = len(names)
     out = {}
@@ -237,7 +249,7 @@ def _reshape(names, pi, pj, cols):
 def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="global", scale_max=True,
                    diag_good=True, include_only=None, alternative="two.sided", continuity=False,
                    check_timing=False, return_matrix=True, colnames=None, device=0, n_gpus=1,
-                   min_abs_cor=None, max_pvalue=None, max_edges=None):
+                   min_abs_cor=None, max_pvalue=None, max_edges=None, p_adjust=None, max_padj=None):
     """All-pairs ICI-Kendall-tau between the columns (samples) of a features x samples matrix.
 
     Returns a dict with `cor`, `raw`, `pvalue`, `taumax`, `completeness` (C x C matrices),
@@ -253,8 +265,17 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
     pairs never pass and raise no warning there.  max_edges: raise IciktError (ERR_LIMIT) when more computed
     pairs than that pass.  The filtered table over several GPUs is _lib.run_edges(..., devices=[...]), which
     returns the same rows as one GPU.
+
+    p_adjust (return_matrix=False): one of R's p.adjust methods ("bonferroni", "holm", "hochberg", "BH" or "fdr",
+    "BY"; not "hommel").  The long table gains a column padj, bit for bit R's p.adjust(pvalue[s1 != s2], method)
+    over the computed pairs of the unfiltered table: every pair, or the include_only pairs, with the diagonal pairs
+    that diag_good=False computes.  The diag_good rows the host appends (p = 0) are not part of that family and get
+    padj = 0.  max_padj keeps the rows with padj <= max_padj, with the same mask rules as max_pvalue (one GPU).  Over
+    all pairs with any bound (min_abs_cor, max_pvalue, max_padj) the adjustment runs on the device window by window
+    with the filter (_lib.run_edges(p_adjust=...)); otherwise the table's p-values are adjusted by _lib.p_adjust.
     """
-    filtered = min_abs_cor is not None or max_pvalue is not None
+    adjusted = _padj_checks(p_adjust, max_padj, return_matrix)
+    filtered = min_abs_cor is not None or max_pvalue is not None or max_padj is not None
     if filtered and return_matrix:
         raise ValueError("`min_abs_cor` and `max_pvalue` select rows of the long table: pass return_matrix=False")
     if filtered and n_gpus > 1:
@@ -312,11 +333,13 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
         out["names"] = names
         return out
     if filtered and all_pairs:  # selected on the device, window by window
+        pk = dict(p_adjust=p_adjust, max_padj=max_padj) if adjusted else {}
         r = _lib.run_edges(data, global_na, min_abs_cor, max_pvalue, scale_max, max_edges or 0,
-                           include_diag=not diag_good, **kw)
+                           include_diag=not diag_good, **pk, **kw)
         run_time = time.perf_counter() - t1
         pi, pj = r["i"], r["j"]
         raw, pvalue, taumax, completeness, cor = (r[k] for k in ("raw", "pvalue", "taumax", "completeness", "cor"))
+        padj = r.get("padj")
     else:
         if all_pairs and n_gpus > 1:  # one call, the pair order sliced over the GPUs inside the library
             r = _lib.run_pairs(data, global_na, include_diag=not diag_good, devices=range(n_gpus), **kw)
@@ -333,20 +356,29 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
             cor = raw / r["max_taumax"]
         else:
             cor = raw.copy()
+        padj = _lib.p_adjust(pvalue, p_adjust, device=device) if adjusted else None
         if filtered:  # include_only: the pair list exists already, the mask runs here
             sel = _edge_mask(cor, pvalue, min_abs_cor, max_pvalue)
+            if max_padj is not None:
+                sel &= padj <= max_padj
             if max_edges and int(sel.sum()) > max_edges:
                 raise _lib.IciktError(_lib.ERR_LIMIT, f"more than max_edges = {max_edges} pairs pass the filter "
                                                       f"({int(sel.sum())})")
             pi, pj, raw, pvalue, taumax, completeness, cor = (
                 v[sel] for v in (pi, pj, raw, pvalue, taumax, completeness, cor))
+            if adjusted:
+                padj = padj[sel]
     if diag_good:  # R/kendalltau.R:374-386 (appended after scaling, never scaled)
         d = np.arange(C, dtype=np.int32)
         dg = n_good / n_good.max()
         dp, dt, dc = np.zeros(C), np.ones(C), n_good / n
         if filtered:
             sel = _edge_mask(dg, dp, min_abs_cor, max_pvalue)
+            if max_padj is not None:
+                sel &= 0.0 <= max_padj
             d, dg, dp, dt, dc = d[sel], dg[sel], dp[sel], dt[sel], dc[sel]
+        if adjusted:
+            padj = np.concatenate([padj, np.zeros(d.size)])
         pi, pj = np.concatenate([pi, d]), np.concatenate([pj, d])
         raw, cor = np.concatenate([raw, dg]), np.concatenate([cor, dg])
         pvalue = np.concatenate([pvalue, dp])
@@ -354,8 +386,10 @@ def ici_kendalltau(data_matrix, global_na=(np.nan, np.inf, 0), perspective="glob
         completeness = np.concatenate([completeness, dc])
     if not return_matrix:
         nm = np.asarray(names, dtype=object)
-        return dict(cor=dict(s1=nm[pi], s2=nm[pj], raw=raw, pvalue=pvalue, taumax=taumax,
-                             completeness=completeness, cor=cor), run_time=run_time, names=names)
+        table = dict(s1=nm[pi], s2=nm[pj], raw=raw, pvalue=pvalue, taumax=taumax, completeness=completeness, cor=cor)
+        if adjusted:
+            table["padj"] = padj
+        return dict(cor=table, run_time=run_time, names=names)
     log.info("Generating the output matrix ...")
     out = _reshape(names, pi, pj, dict(cor=cor, raw=raw, pvalue=pvalue, taumax=taumax,
                                         completeness=completeness))
@@ -422,7 +456,8 @@ def _names_by_index(names):
 
 def ici_kendalltau_cross(x, y, global_na=(np.nan, np.inf, 0), perspective="global", scale_max=True,
                          alternative="two.sided", continuity=False, return_matrix=True, min_abs_cor=None,
-                         max_pvalue=None, max_edges=None, xnames=None, ynames=None, device=0, n_gpus=1):
+                         max_pvalue=None, max_edges=None, xnames=None, ynames=None, device=0, n_gpus=1,
+                         p_adjust=None, max_padj=None):
     """ICI-Kendall-tau of every column (sample) of `x` with every column of `y`, both features x samples with the
     same features: query samples against a reference panel, two batches, two feature sets on the same samples.
 
@@ -438,10 +473,15 @@ def ici_kendalltau_cross(x, y, global_na=(np.nan, np.inf, 0), perspective="globa
     table; max_edges raises IciktError (ERR_LIMIT) when more pairs pass.  One GPU: n_gpus must be 1.  The same
     results over several GPUs are _lib.run_cross(x, y, devices=[...]) and _lib.run_cross_edges(..., devices=[...]),
     which return bit for bit what one GPU returns.
+
+    p_adjust / max_padj (return_matrix=False) as in ici_kendalltau: the long table gains padj, bit for bit R's
+    p.adjust(pvalue, method) over all Cx x Cy pairs; with any bound the adjustment runs on the device with the filter
+    (_lib.run_cross_edges(p_adjust=...)), otherwise _lib.p_adjust adjusts the table's p-values.
     """
     if n_gpus != 1:
         raise ValueError("the cross calls run on one GPU: n_gpus must be 1")
-    filtered = min_abs_cor is not None or max_pvalue is not None
+    adjusted = _padj_checks(p_adjust, max_padj, return_matrix)
+    filtered = min_abs_cor is not None or max_pvalue is not None or max_padj is not None
     if filtered and return_matrix:
         raise ValueError("`min_abs_cor` and `max_pvalue` select rows of the long table: pass return_matrix=False")
     if max_edges is not None and not filtered:
@@ -453,12 +493,15 @@ def ici_kendalltau_cross(x, y, global_na=(np.nan, np.inf, 0), perspective="globa
     log.info("Running correlations ...")
     t1 = time.perf_counter()
     if filtered:
-        r = _lib.run_cross_edges(x, y, global_na, min_abs_cor, max_pvalue, scale_max, max_edges or 0, **kw)
+        pk = dict(p_adjust=p_adjust, max_padj=max_padj) if adjusted else {}
+        r = _lib.run_cross_edges(x, y, global_na, min_abs_cor, max_pvalue, scale_max, max_edges or 0, **pk, **kw)
         run_time = time.perf_counter() - t1
         xn, yn = np.asarray(xnames, dtype=object), np.asarray(ynames, dtype=object)
-        return dict(cor=dict(s1=xn[r["i"]], s2=yn[r["j"]], raw=r["raw"], pvalue=r["pvalue"], taumax=r["taumax"],
-                             completeness=r["completeness"], cor=r["cor"]),
-                    run_time=run_time, xnames=xnames, ynames=ynames)
+        table = dict(s1=xn[r["i"]], s2=yn[r["j"]], raw=r["raw"], pvalue=r["pvalue"], taumax=r["taumax"],
+                     completeness=r["completeness"], cor=r["cor"])
+        if adjusted:
+            table["padj"] = r["padj"]
+        return dict(cor=table, run_time=run_time, xnames=xnames, ynames=ynames)
     r = _lib.run_cross(x, y, global_na, **kw)
     run_time = time.perf_counter() - t1
     _warn_status(r["status"])
@@ -468,6 +511,8 @@ def ici_kendalltau_cross(x, y, global_na=(np.nan, np.inf, 0), perspective="globa
         xn, yn = np.asarray(xnames, dtype=object), np.asarray(ynames, dtype=object)
         table = dict(s1=np.repeat(xn, cy), s2=np.tile(yn, cx))
         table.update((k, cols[k]) for k in ("raw", "pvalue", "taumax", "completeness", "cor"))
+        if adjusted:
+            table["padj"] = _lib.p_adjust(r["pvalue"], p_adjust, device=device)
         return dict(cor=table, run_time=run_time, xnames=xnames, ynames=ynames)
     out = {k: cols[k].reshape(cx, cy) for k in _lib.MATRIX_NAMES}
     out.update(xnames=xnames, ynames=ynames, run_time=run_time)

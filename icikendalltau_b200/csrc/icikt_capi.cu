@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <memory>
 #include <mutex>
 #include <new>
@@ -22,6 +23,7 @@
 #include "icikt_cross.cuh"
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
+#include "icikt_padj.cuh"
 #include "icikt_topk.cuh"
 
 using namespace icikt;
@@ -1691,6 +1693,8 @@ struct icikt_edges {
   std::vector<EdgeRow> rows;
   std::vector<double> cor;
   int32_t j_offset = 0;  // a cross call's Cx: rows hold j as the matrix column of [X | Y], icikt_edges_copy gives Y's
+  std::vector<double> padj;  // the _padj calls: the adjusted p-value of every row
+  int64_t n_tests = -1;      // ... and m, the non-NaN p-values of the family; -1 without adjustment
 };
 
 // Pairs per window of the filtered calls, edges, top-k and cross (ICIKT_EDGE_WINDOW, at most 2^30).  The default 2^26
@@ -1980,6 +1984,68 @@ static int finish_walk(icikt_plan* p, const WalkTotals& tot, float d2h_ms, icikt
   return ICIKT_OK;
 }
 
+// ---- adjusted p-values (the _padj edge calls): every walker keeps the count of the non-NaN p-values of its slice and
+// the keys of its candidates, the p-values <= the candidate bound (icikt_padj.cuh: a prefix of the ascending order
+// that holds every row whose adjusted value can pass).  The buffer grows geometrically; it always has room for the two
+// windows whose counts the host has not read back yet.
+struct PadjPart {
+  int device = -1;
+  unsigned long long* d_cnt = nullptr;   // [2]: non-NaN p-values, candidates
+  unsigned long long* h_cnt = nullptr;   // pinned [2][2]: the readback of d_cnt, per window buffer
+  unsigned long long* d_keys = nullptr;  // [cap]
+  int64_t cap = 0, known = 0;            // capacity; candidates as of the last readback
+  int64_t m = 0, K = 0;                  // after the walk: non-NaN p-values and candidates
+  double bound = 0.0;                    // the candidate bound (NaN: every non-NaN p-value)
+  PadjPart() = default;
+  PadjPart(const PadjPart&) = delete;
+  PadjPart& operator=(const PadjPart&) = delete;
+  ~PadjPart() { release(); }
+  void release() {
+    if (device < 0) return;
+    cudaSetDevice(device);
+    cudaFree(d_cnt);
+    cudaFree(d_keys);
+    if (h_cnt) cudaFreeHost(h_cnt);
+    d_cnt = d_keys = h_cnt = nullptr;
+    device = -1;
+    cap = 0;
+  }
+};
+
+// room in a's buffer for `more` candidates beyond those last read back (set up on p's device at the first window)
+static int padj_room(icikt_plan* p, PadjPart& a, int64_t more) {
+  if (a.device < 0) {
+    a.device = p->device;
+    ECK(dmalloc(&a.d_cnt, 2));
+    ECK(cudaMallocHost(reinterpret_cast<void**>(&a.h_cnt), 4 * sizeof(unsigned long long)));
+    std::memset(a.h_cnt, 0, 4 * sizeof(unsigned long long));
+    CK(cudaMemsetAsync(a.d_cnt, 0, 2 * sizeof(unsigned long long), p->stream));
+  }
+  if (a.known + more <= a.cap) return ICIKT_OK;
+  CK(cudaStreamSynchronize(p->stream));  // the windows in flight append to the old buffer
+  unsigned long long now[2];
+  CK(cudaMemcpy(now, a.d_cnt, sizeof(now), cudaMemcpyDeviceToHost));
+  a.known = (int64_t)now[1];
+  const int64_t cap = std::max(2 * a.cap, a.known + more);
+  unsigned long long* keys = nullptr;
+  if (dmalloc(&keys, (size_t)cap) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ICIKT_ERR_ALLOC, "device allocation for " + std::to_string(cap) + " p-value candidates failed (" +
+                                     std::to_string(a.known) + " held)");
+  }
+  if (a.known) {
+    const cudaError_t e = cudaMemcpy(keys, a.d_keys, sizeof(unsigned long long) * (size_t)a.known, cudaMemcpyDeviceToDevice);
+    if (e != cudaSuccess) {
+      cudaFree(keys);
+      return cuda_fail(e, "p-value candidates");
+    }
+  }
+  cudaFree(a.d_keys);
+  a.d_keys = keys;
+  a.cap = cap;
+  return ICIKT_OK;
+}
+
 // The rows all walkers of one filtered call hold, for max_edges: one walker on one device, one per device in the
 // multi-device call.  A walker that takes the sum over the limit raises `stop`, and the others fail at their next
 // window boundary.
@@ -1999,7 +2065,8 @@ static int edge_limit_fail(const icikt_edge_filter& f, int64_t held, const std::
 // stay a superset of the final edges).  The plan's edge buffers hold windows of W pairs.
 template <class Order>
 static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter& f, int64_t first, int64_t last,
-                     int64_t W, std::vector<EdgeRow>& rows, EdgeHeld& held, WalkTotals& tot, float& d2h_ms) {
+                     int64_t W, std::vector<EdgeRow>& rows, EdgeHeld& held, WalkTotals& tot, float& d2h_ms,
+                     PadjPart* adj = nullptr) {
   const double t = f.min_abs_cor;
   const bool scale = f.scale_max != 0;
   const bool retrim = scale && t == t;
@@ -2028,6 +2095,12 @@ static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter&
     if (l < 0) return launch_fail("edge selection kernels");
     tot.launches += l;
     CK(cudaMemcpyAsync(p->h_estat + 2 * b, p->d_etotal + b, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    if (adj) {  // the window's non-NaN count and candidates, in the epilogue's time
+      const int r = padj_room(p, *adj, 2 * W);
+      if (r != ICIKT_OK) return r;
+      CK(padj_candidates(p->d_p, n_slots, adj->bound, adj->d_cnt, adj->d_keys, p->stream));
+      CK(cudaMemcpyAsync(adj->h_cnt + 2 * b, adj->d_cnt, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    }
     return ICIKT_OK;
   };
 
@@ -2035,6 +2108,7 @@ static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter&
     if (held.stop) return edge_limit_fail(f, held.total, " held when another device reached the limit");
     const unsigned long long cnt = p->h_estat[2 * b];
     const unsigned long long bits = tot.bits;
+    if (adj) adj->known = std::max<int64_t>(adj->known, (int64_t)adj->h_cnt[2 * b + 1]);
     const size_t before = rows.size();
     if (cnt) {
       const size_t old = rows.size();
@@ -2064,18 +2138,30 @@ static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter&
     return ICIKT_OK;
   };
 
-  return walk_windows(p, order, first, last, W, tot, select, collect);
+  const int rc = walk_windows(p, order, first, last, W, tot, select, collect);
+  if (rc != ICIKT_OK || !adj || adj->device < 0) return rc;
+  unsigned long long now[2];
+  CK(cudaStreamSynchronize(p->stream));
+  CK(cudaMemcpy(now, adj->d_cnt, sizeof(now), cudaMemcpyDeviceToHost));
+  adj->m = (int64_t)now[0];
+  adj->K = (int64_t)now[1];
+  return ICIKT_OK;
 }
 
 // The end of the filtered call, on one device or several: the rows held, in pair order, get the exact predicate with
-// the final maximum M, the max_edges check and cor.
-static int edge_result(icikt_edges* res, const icikt_edge_filter& f, double M) {
+// the final maximum M, then `adjust` (the _padj calls: adjusted p-values and their trim), the max_edges check and cor.
+static int edge_result(icikt_edges* res, const icikt_edge_filter& f, double M,
+                       const std::function<int(icikt_edges*)>& adjust = nullptr) {
   std::vector<EdgeRow>& rows = res->rows;
   const double t = f.min_abs_cor;
   const bool scale = f.scale_max != 0;
   if (scale && t == t)
     rows.erase(std::remove_if(rows.begin(), rows.end(), [&](const EdgeRow& r) { return !edge_keep_final(r.raw, t, true, M); }),
                rows.end());
+  if (adjust) {
+    const int rc = adjust(res);
+    if (rc != ICIKT_OK) return rc;
+  }
   if (f.max_edges > 0 && (int64_t)rows.size() > f.max_edges) return edge_limit_fail(f, (int64_t)rows.size(), "");
   try {
     res->cor.resize(rows.size());
@@ -2835,18 +2921,154 @@ int no_pairs(double* max_taumax, icikt_timings* timings) {
   return ICIKT_OK;
 }
 
+// The adjusted p-values of the rows held (the _padj calls), once every worker has walked its slice: m is the sum of
+// the workers' non-NaN counts; their candidates are gathered on devices[0] (the same device: a device copy; peer
+// access between all devices: peer copies; otherwise through pinned host memory), sorted and scanned there once, and
+// every row looks its value up there.  m <= 1 leaves the p-values as they are (p.adjust).  Then the rows with
+// padj > max_padj go.  dev_ms receives the device time of the gather, sort, scan and lookup.
+using DevPtr = std::unique_ptr<void, cudaError_t (*)(void*)>;
+
+int padj_gather(const MultiJob& J, std::vector<PadjPart>& parts, int dev, int64_t K, unsigned long long** all, DevPtr& own) {
+  PadjPart& first = parts[0];
+  int64_t at = 0;
+  size_t k0 = 0;
+  if (first.device == dev && first.cap >= K) {  // the first worker's buffer takes the others' candidates
+    *all = first.d_keys;
+    at = first.K;
+    k0 = 1;
+  } else {
+    if (dmalloc(all, (size_t)K) != cudaSuccess) {
+      cudaGetLastError();
+      return fail(ICIKT_ERR_ALLOC, "device allocation for the " + std::to_string(K) + " p-value candidates failed");
+    }
+    own.reset(*all);
+  }
+  unsigned long long* stage = nullptr;
+  const size_t chunk = 4u << 20;  // keys per staged piece (32 MB)
+  int rc = ICIKT_OK;
+  for (size_t k = k0; k < parts.size() && rc == ICIKT_OK; ++k) {
+    PadjPart& pt = parts[k];
+    const size_t bytes = sizeof(unsigned long long) * (size_t)pt.K;
+    cudaError_t e = cudaSuccess;
+    if (!pt.K) continue;
+    if (pt.device == dev) {
+      e = cudaMemcpy(*all + at, pt.d_keys, bytes, cudaMemcpyDeviceToDevice);
+    } else if (J.peers_ok) {
+      e = cudaMemcpyPeer(*all + at, dev, pt.d_keys, pt.device, bytes);
+    } else {
+      if (!stage && (e = cudaMallocHost(reinterpret_cast<void**>(&stage), sizeof(unsigned long long) * chunk)) != cudaSuccess)
+        break;
+      for (int64_t o = 0; o < pt.K && e == cudaSuccess; o += (int64_t)chunk) {
+        const size_t b = sizeof(unsigned long long) * std::min<size_t>(chunk, (size_t)(pt.K - o));
+        if ((e = cudaSetDevice(pt.device)) == cudaSuccess) e = cudaMemcpy(stage, pt.d_keys + o, b, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && (e = cudaSetDevice(dev)) == cudaSuccess)
+          e = cudaMemcpy(*all + at + o, stage, b, cudaMemcpyHostToDevice);
+      }
+      cudaSetDevice(dev);
+    }
+    if (e != cudaSuccess) rc = cuda_fail(e, "gathering the p-value candidates");
+    at += pt.K;
+    pt.release();
+    cudaSetDevice(dev);
+  }
+  if (stage) cudaFreeHost(stage);
+  return rc;
+}
+
+int padj_finish(const MultiJob& J, std::vector<PadjPart>& parts, const icikt_padj_filter& a, icikt_edges* res,
+                float* dev_ms) {
+  int64_t m = 0, K = 0;
+  for (const PadjPart& pt : parts) {
+    m += pt.m;
+    K += pt.K;
+  }
+  res->n_tests = m;
+  std::vector<EdgeRow>& rows = res->rows;
+  std::vector<double>& padj = res->padj;
+  const int64_t R = (int64_t)rows.size();
+  try {
+    padj.resize((size_t)R);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the adjusted p-values");
+  }
+  *dev_ms = 0.f;
+  if (m <= 1) {
+    for (int64_t r = 0; r < R; ++r) padj[(size_t)r] = rows[(size_t)r].pvalue;
+  } else if (R > 0) {
+    const int dev = J.device_of(0);
+    CK(cudaSetDevice(dev));
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    CK(cudaEventCreate(&ev[0]));
+    std::unique_ptr<CUevent_st, cudaError_t (*)(cudaEvent_t)> e0(ev[0], cudaEventDestroy);
+    CK(cudaEventCreate(&ev[1]));
+    std::unique_ptr<CUevent_st, cudaError_t (*)(cudaEvent_t)> e1(ev[1], cudaEventDestroy);
+    CK(cudaEventRecord(ev[0], 0));
+    unsigned long long* all = nullptr;
+    DevPtr own(nullptr, cudaFree);
+    int rc = padj_gather(J, parts, dev, K, &all, own);
+    if (rc != ICIKT_OK) return rc;
+    const double q = a.method == ICIKT_PADJ_BY ? padj_by_q(m) : 0.0;
+    unsigned long long *alt = nullptr, *sorted = nullptr;
+    double *vals = nullptr, *d_p = nullptr;
+    if (dmalloc(&alt, (size_t)K) != cudaSuccess || dmalloc(&d_p, 2 * (size_t)R) != cudaSuccess) {
+      cudaGetLastError();
+      cudaFree(alt);
+      return fail(ICIKT_ERR_ALLOC, "device allocation for sorting " + std::to_string(K) + " p-value candidates failed");
+    }
+    DevPtr own_alt(alt, cudaFree), own_p(d_p, cudaFree);
+    std::vector<double> p;
+    try {
+      p.resize((size_t)R);
+    } catch (const std::bad_alloc&) {
+      return fail(ICIKT_ERR_ALLOC, "out of host memory for the adjusted p-values");
+    }
+    for (int64_t r = 0; r < R; ++r) p[(size_t)r] = rows[(size_t)r].pvalue;
+    CK(padj_sort_scan(all, alt, K, m, a.method, q, &sorted, &vals, 0));
+    CK(cudaMemcpy(d_p, p.data(), sizeof(double) * (size_t)R, cudaMemcpyHostToDevice));
+    CK(padj_lookup(sorted, vals, K, a.method, d_p, R, d_p + R, 0));
+    CK(cudaMemcpy(padj.data(), d_p + R, sizeof(double) * (size_t)R, cudaMemcpyDeviceToHost));
+    CK(cudaEventRecord(ev[1], 0));
+    CK(cudaEventSynchronize(ev[1]));
+    *dev_ms = ev_ms(ev[0], ev[1]);
+  }
+  const double t = a.max_padj;
+  if (t == t) {
+    size_t w = 0;
+    for (size_t r = 0; r < rows.size(); ++r)
+      if (padj[r] <= t) {
+        rows[w] = rows[r];
+        padj[w++] = padj[r];
+      }
+    rows.resize(w);
+    padj.resize(w);
+  }
+  return ICIKT_OK;
+}
+
 // The filtered call over the devices of J, its arguments checked: every worker walks its slice against the shared
 // EdgeHeld, then the rows are joined in worker order (the slices are contiguous and in order, so are the rows; the
-// first worker's rows are moved, not copied) and edge_result trims them with the final maximum.
-int edges_run(MultiJob& J, const icikt_edge_filter& f, icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+// first worker's rows are moved, not copied) and edge_result trims them with the final maximum.  With `adjust`
+// (the _padj calls), every worker also keeps its candidates, and padj_finish gives the rows their adjusted values.
+int edges_run(MultiJob& J, const icikt_edge_filter& f0, icikt_edges** out, double* max_taumax, icikt_timings* timings,
+              const icikt_padj_filter* adjust = nullptr) {
   int rc = select_device(J.device_of(0));
   if (rc != ICIKT_OK) return rc;
   std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
   if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
   res->j_offset = J.y ? (int32_t)J.src.C : 0;
+  if (adjust) res->n_tests = 0;
   if (J.ptot == 0) {  // one column, no diagonal: nothing to compute
     *out = res.release();
     return no_pairs(max_taumax, timings);
+  }
+  // The candidate bound: every row with padj <= max_padj has p <= max_padj (icikt_padj.cuh).  A max_padj >= 1 keeps
+  // every row, as does NaN.  The rows take it as one more p-value bound.
+  icikt_edge_filter f = f0;
+  std::vector<PadjPart> parts(adjust ? (size_t)J.n_devices : 0);
+  if (adjust) {
+    const double b = adjust->max_padj < 1.0 ? adjust->max_padj : std::nan("");
+    for (PadjPart& pt : parts) pt.bound = b;
+    if (b == b && !(f.max_pvalue <= b)) f.max_pvalue = b;
   }
   std::vector<MultiWork> work;
   std::vector<std::vector<EdgeRow>> rows((size_t)J.n_devices);
@@ -2865,7 +3087,8 @@ int edges_run(MultiJob& J, const icikt_edge_filter& f, icikt_edges** out, double
       r = ensure_edge_buffers(p, p->P);
       if (r == ICIKT_OK)
         r = with_order(J, p, [&](const auto& order) {
-          return edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms);
+          return edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms,
+                           adjust ? &parts[(size_t)k] : nullptr);
         });
       if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
       bits[(size_t)k] = tot.bits;
@@ -2886,8 +3109,14 @@ int edges_run(MultiJob& J, const icikt_edge_filter& f, icikt_edges** out, double
     std::vector<EdgeRow>().swap(rows[k]);
   }
   const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
-  rc = edge_result(res.get(), f, M);
+  float padj_ms = 0.f;
+  rc = edge_result(res.get(), f, M, adjust ? [&](icikt_edges* e) { return padj_finish(J, parts, *adjust, e, &padj_ms); }
+                                           : std::function<int(icikt_edges*)>());
   if (rc != ICIKT_OK) return rc;
+  if (timings) {  // the adjustment's device work counts as epilogue, and the call's device work ends with it
+    timings->epilogue_ms += padj_ms;
+    timings->total_ms += padj_ms;
+  }
   if (max_taumax) *max_taumax = M;
   *out = res.release();
   return ICIKT_OK;
@@ -3147,6 +3376,53 @@ int cross_topk_impl(const icikt_input* x, const icikt_input* y, int64_t n, const
   return topk_run(J, K, by, scale_max != 0, c_lo, c_hi, sides, max_taumax, timings);
 }
 
+// ---- the filtered calls with adjusted p-values (_padj): the all-pairs or cross job of the edges calls, with adjust
+
+int check_padj_method(int32_t method) {
+  if (method < ICIKT_PADJ_BONFERRONI || method > ICIKT_PADJ_BY)
+    return fail(ICIKT_ERR_BAD_ARG, "method must be one of ICIKT_PADJ_BONFERRONI .. ICIKT_PADJ_BY (Hommel is not offered)");
+  return ICIKT_OK;
+}
+
+int check_padj(const icikt_padj_filter* a) {
+  if (!a) return fail(ICIKT_ERR_BAD_ARG, "adjust is NULL");
+  const int rc = check_padj_method(a->method);
+  if (rc != ICIKT_OK) return rc;
+  if (a->reserved != 0) return fail(ICIKT_ERR_BAD_ARG, "adjust->reserved must be 0");
+  return ICIKT_OK;
+}
+
+int edges_padj_impl(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na, const icikt_opts& o,
+                    const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filter,
+                    const icikt_padj_filter* adjust, icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  ColumnSource s;
+  int rc = check_filter_args(filter, out);
+  if (rc == ICIKT_OK) rc = check_padj(adjust);
+  if (rc == ICIKT_OK) rc = n < 1 ? fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1") : cross_source(x, "x", n, &s);
+  if (rc == ICIKT_OK) rc = check_window_args(s, n, s.C, global_na, n_global_na, o);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  MultiJob J(n_devices);
+  J.src = s; J.n = n; J.C = s.C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.ptot = tri_pairs(s.C) + (o.include_diag ? s.C : 0);
+  return edges_run(J, *filter, out, max_taumax, timings, adjust);
+}
+
+int cross_edges_padj_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                          int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices,
+                          const icikt_edge_filter* filter, const icikt_padj_filter* adjust, icikt_edges** out,
+                          double* max_taumax, icikt_timings* timings) {
+  ColumnSource sx, sy;
+  int rc = check_filter_args(filter, out);
+  if (rc == ICIKT_OK) rc = check_padj(adjust);
+  if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  MultiJob J(n_devices);
+  cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
+  return edges_run(J, *filter, out, max_taumax, timings, adjust);
+}
+
 }  // namespace
 
 extern "C" {
@@ -3360,6 +3636,76 @@ int icikt_pnorm_device(const double* z, int64_t n, int32_t lower_tail, double* o
   cudaFree(dz);
   cudaFree(dout);
   if (e != cudaSuccess) return cuda_fail(e, "pnorm");
+  return ICIKT_OK;
+}
+
+
+int icikt_all_pairs_edges_padj(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                               const icikt_opts* opts, const icikt_edge_filter* filter, const icikt_padj_filter* adjust,
+                               icikt_edges** out, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return edges_padj_impl(x, n, global_na, n_global_na, o, &o.device, 1, filter, adjust, out, max_taumax, timings);
+}
+
+int icikt_all_pairs_edges_padj_multi(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                     const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                     const icikt_edge_filter* filter, const icikt_padj_filter* adjust, icikt_edges** out,
+                                     double* max_taumax, icikt_timings* timings) {
+  return edges_padj_impl(x, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filter, adjust, out,
+                         max_taumax, timings);
+}
+
+int icikt_cross_edges_padj(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
+                           const icikt_padj_filter* adjust, icikt_edges** out, double* max_taumax,
+                           icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return cross_edges_padj_impl(x, y, n, global_na, n_global_na, o, &o.device, 1, filter, adjust, out, max_taumax,
+                               timings);
+}
+
+int icikt_cross_edges_padj_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                                 int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                 const icikt_edge_filter* filter, const icikt_padj_filter* adjust, icikt_edges** out,
+                                 double* max_taumax, icikt_timings* timings) {
+  return cross_edges_padj_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filter,
+                               adjust, out, max_taumax, timings);
+}
+
+int icikt_edges_copy_padj(const icikt_edges* e, double* padj) {
+  if (!e) return fail(ICIKT_ERR_BAD_ARG, "edges is NULL");
+  if (e->n_tests < 0) return fail(ICIKT_ERR_BAD_ARG, "the result holds no adjusted p-values (not from a _padj call)");
+  if (!padj && !e->padj.empty()) return fail(ICIKT_ERR_BAD_ARG, "padj is NULL");
+  if (!e->padj.empty()) std::memcpy(padj, e->padj.data(), sizeof(double) * e->padj.size());
+  return ICIKT_OK;
+}
+
+int64_t icikt_edges_n_tests(const icikt_edges* e) { return e ? e->n_tests : -1; }
+
+int icikt_p_adjust(const double* p, int64_t m, int32_t method, int32_t device, double* out, int64_t* n_tests) {
+  if (m < 0) return fail(ICIKT_ERR_BAD_ARG, "m must be >= 0");
+  if (m > 0 && (!p || !out)) return fail(ICIKT_ERR_BAD_ARG, "p and out must not be NULL");
+  int rc = check_padj_method(method);
+  if (rc == ICIKT_OK) rc = select_device(device);
+  if (rc != ICIKT_OK) return rc;
+  int64_t mm = 0;
+  if (m > 0) {
+    double* d = nullptr;
+    if (dmalloc(&d, 2 * (size_t)m) != cudaSuccess) {
+      cudaGetLastError();
+      return fail(ICIKT_ERR_ALLOC, "device allocation for " + std::to_string(m) + " p-values failed");
+    }
+    cudaError_t e = cudaMemcpy(d, p, sizeof(double) * (size_t)m, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = padj_array(d, m, method, d + m, &mm, nullptr, 0);
+    if (e == cudaSuccess) e = cudaMemcpy(out, d + m, sizeof(double) * (size_t)m, cudaMemcpyDeviceToHost);
+    cudaFree(d);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return e == cudaErrorMemoryAllocation ? fail(ICIKT_ERR_ALLOC, "device allocation for p.adjust failed")
+                                            : cuda_fail(e, "p.adjust");
+    }
+  }
+  if (n_tests) *n_tests = mm;
   return ICIKT_OK;
 }
 

@@ -259,6 +259,24 @@ struct TopkDeviceMerge {
 };
 int launch_topk_device_merge(const TopkDeviceMerge& m, cudaStream_t stream);
 
+// R's p.adjust on the device (icikt_padj.cu, arithmetic in icikt_padj.cuh).  Each returns the first CUDA error.
+// counts[0] += the non-NaN values of p[0, n); the keys (padj_key) of those <= bound (NaN: all) are appended at
+// keys[counts[1]++], which the caller has made room for.
+cudaError_t padj_candidates(const double* p, int64_t n, double bound, unsigned long long* counts,
+                            unsigned long long* keys, cudaStream_t stream);
+// sorts keys[0, K) (alt: a second buffer of K), then the running max / min of the per-rank values over m tests; on
+// return *sorted is the buffer that holds the sorted keys and *vals the other one, holding the scanned values.
+// Synchronises the stream.
+cudaError_t padj_sort_scan(unsigned long long* keys, unsigned long long* alt, int64_t K, int64_t m, int method,
+                           double q, unsigned long long** sorted, double** vals, cudaStream_t stream);
+// out[r] = the adjusted value of p[r], every p[r] one of the K sorted keys
+cudaError_t padj_lookup(const unsigned long long* sorted, const double* vals, int64_t K, int method, const double* p,
+                        int64_t R, double* out, cudaStream_t stream);
+// p.adjust(p[0, m), method) into out (device arrays); *n_tests = the non-NaN values; q_ms (may be NULL): the host
+// time of BY's sum.  Synchronises the stream.
+cudaError_t padj_array(const double* p, int64_t m, int method, double* out, int64_t* n_tests, double* q_ms,
+                       cudaStream_t stream);
+
 int launch_pnorm(const double* d_z, int64_t n, int lower, double* d_out, cudaStream_t stream);
 
 int64_t tiled_max_n();

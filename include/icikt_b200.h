@@ -458,6 +458,70 @@ int icikt_cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n
                            int32_t k, int32_t by, int32_t scale_max, const icikt_topk_lists* x_side,
                            const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings);
 
+/* ---- filtered calls with p-values adjusted over every pair: R's p.adjust(p_all, method), computed on the device window
+ * by window without holding P of anything, where p_all is the per-pair p-value array of icikt_all_pairs /
+ * icikt_cross_pairs.  Methods are R's bonferroni, holm, hochberg, BH (fdr) and BY; Hommel is not offered (its adjusted
+ * values depend on the whole order, not on a prefix).
+ *
+ *   - Family: every pair of the call's order whose p-value is not NaN, whatever its status: the combn order plus the
+ *     diagonal pairs when include_diag is set, or the Cx * Cy cross order.  m, their number, is what p.adjust's n is
+ *     after it drops the NAs.  The family does not depend on min_abs_cor or max_pvalue.
+ *   - Row predicate: that of icikt_all_pairs_edges / icikt_cross_edges AND (isnan(max_padj) || padj <= max_padj).
+ *     Rows, their order, every existing field and max_taumax are bit for bit what those calls return for the same
+ *     pairs; padj (icikt_edges_copy_padj) is bit for bit p.adjust(p_all, method) at the row's pair.
+ *   - Exactness without every p-value: each multiplier of p.adjust is >= 1 after rounding, so padj >= p, and the
+ *     p-values <= max_padj are a prefix of the ascending order whose adjusted values <= max_padj depend only on that
+ *     prefix and on m.  Each device keeps one 8-byte key per pair with p <= max_padj (every non-NaN p-value when
+ *     max_padj is NaN or >= 1: 8 B per pair) and a count of the non-NaN p-values; after the last window the keys are
+ *     gathered on devices[0] (peer copies when every pair of devices has peer access, otherwise through pinned host
+ *     memory), sorted and scanned once, and every row finds its value by a binary search of its p-value.  BY's
+ *     q = sum(1/(1:m)) is summed on the host in long double, as R's sum does (m steps).  m <= 1 leaves padj = p.
+ *   - Refused with ICIKT_ERR_BAD_ARG before any device is touched: whatever the matching edges call refuses, a NULL
+ *     adjust, a method out of range, reserved != 0.  The all-pairs calls take the matrix as an icikt_input, dense or
+ *     CSC, whose messages name it matrix x.
+ *   - max_edges counts the rows held, as in the edges calls (rows are held only when p <= max_padj too); the final
+ *     count is taken after the trim with padj.
+ *   - timings as in the edges calls; the candidates' pass, the gather, sort, scan and lookup are counted in
+ *     epilogue_ms, and total_ms ends with the lookup.  The _multi twins take (devices, n_devices) after opts, as the
+ *     edges multi calls, and return bit for bit the single-device result (padj depends only on the p-values and m). */
+#define ICIKT_PADJ_BONFERRONI 1
+#define ICIKT_PADJ_HOLM 2
+#define ICIKT_PADJ_HOCHBERG 3
+#define ICIKT_PADJ_BH 4 /* R's "BH" and "fdr" */
+#define ICIKT_PADJ_BY 5
+
+typedef struct icikt_padj_filter {
+  int32_t method;   /* ICIKT_PADJ_*                                  */
+  int32_t reserved; /* 0                                             */
+  double max_padj;  /* NaN: no condition on the adjusted p-value     */
+} icikt_padj_filter;
+
+/* R's p.adjust(p[0..m), method) on the device: NaN entries are dropped from the family and stay as they are (their
+ * bits), *n_tests (may be NULL) receives the number of non-NaN entries, and fewer than two of them leave p unchanged.
+ * -0.0 counts as +0.0.  p and out may be NULL when m == 0.  Refused with ICIKT_ERR_BAD_ARG: m < 0, NULL p / out with
+ * m > 0, a method out of range.  Device memory: about 56 B per entry. */
+int icikt_p_adjust(const double* p, int64_t m, int32_t method, int32_t device, double* out, int64_t* n_tests);
+
+int icikt_all_pairs_edges_padj(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                               const icikt_opts* opts, const icikt_edge_filter* filter, const icikt_padj_filter* adjust,
+                               icikt_edges** out, double* max_taumax, icikt_timings* timings);
+int icikt_all_pairs_edges_padj_multi(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                     const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                     const icikt_edge_filter* filter, const icikt_padj_filter* adjust, icikt_edges** out,
+                                     double* max_taumax, icikt_timings* timings);
+int icikt_cross_edges_padj(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filter,
+                           const icikt_padj_filter* adjust, icikt_edges** out, double* max_taumax,
+                           icikt_timings* timings);
+int icikt_cross_edges_padj_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                                 int32_t n_global_na, const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                 const icikt_edge_filter* filter, const icikt_padj_filter* adjust, icikt_edges** out,
+                                 double* max_taumax, icikt_timings* timings);
+/* the adjusted p-values of a _padj result into padj[icikt_edges_count(e)]; ICIKT_ERR_BAD_ARG for a result without */
+int icikt_edges_copy_padj(const icikt_edges* e, double* padj);
+/* m of a _padj result; -1 for NULL or a result without adjustment */
+int64_t icikt_edges_n_tests(const icikt_edges* e);
+
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
  * pay the copies.  A plan is bound to one device and is not thread-safe.            */
