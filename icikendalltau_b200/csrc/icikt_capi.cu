@@ -1456,89 +1456,42 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
 
 // all pairs of a matrix this large go through the pipelined call (ICIKT_PIPELINE_MIN_BYTES, default 32 MB of
 // input; ICIKT_NO_PIPELINE=1 switches it off)
-static bool want_staged(int64_t n, int64_t C, const icikt_opts& o, bool all_pairs) {
-  if (!all_pairs || o.pair_lo != 0 || o.pair_hi != 0 || o.kernel != ICIKT_KERNEL_TILED) return false;
-  if (std::getenv("ICIKT_NO_PIPELINE")) return false;
+static bool want_staged(int64_t n, int64_t C, const icikt_opts& o) {
+  if (o.kernel != ICIKT_KERNEL_TILED || std::getenv("ICIKT_NO_PIPELINE")) return false;
   const size_t min_bytes = env_bytes("ICIKT_PIPELINE_MIN_BYTES", 32u << 20);
   return C >= 128 && sizeof(double) * (size_t)n * (size_t)C >= min_bytes;
 }
 
-// One cached plan for the one-shot entry points (all-pairs shape only).
+// The cached plans: the per-pair and matrix calls' (one worker: g_cached, worker k of several: g_cached_multi[k]) and
+// the windowed calls' (g_cached_edges, g_cached_wmulti[k]; their pair buffers hold one window).
 static icikt_plan* g_cached = nullptr;
-static icikt_plan* g_cached_multi[64] = {};  // one slot per worker of icikt_all_pairs_multi
-static icikt_plan* g_cached_edges = nullptr;    // a windowed call's on one device (its pair buffers hold one window)
-static icikt_plan* g_cached_wmulti[kMaxMatrixDevices] = {};  // one slot per worker of a windowed call on several
+static icikt_plan* g_cached_multi[64] = {};
+static icikt_plan* g_cached_edges = nullptr;
+static icikt_plan* g_cached_wmulti[kMaxMatrixDevices] = {};
 static std::mutex g_cache_mu;
 
-static bool cache_matches(const icikt_plan* p, int64_t n, int64_t C, const icikt_opts& o, bool staged) {
-  return p && p->staged == staged && p->n == n && p->C == C && p->opts.device == o.device && p->opts.kernel == o.kernel &&
-         p->opts.include_diag == o.include_diag && p->opts.pair_lo == o.pair_lo &&
-         p->opts.pair_hi == o.pair_hi && p->want_counts == (o.want_counts != 0);
-}
-
-// a cached plan taken by a call: the options that do not shape the plan are the call's
-static void reuse_plan(icikt_plan* p, const icikt_opts& o) {
-  p->opts.perspective = o.perspective;
-  p->opts.alternative = o.alternative;
-  p->opts.continuity = o.continuity;
-  p->opts.na_inf = o.na_inf;
-}
-
-struct MatrixOut {  // the download step of one_shot as matrices instead of per-pair arrays
-  int32_t scale_max, diag_good;
-  const int32_t* n_good;
-  double* cor;
-  int64_t* status_counts;
-};
-
-static int one_shot(const ColumnSource& s, int64_t n, int64_t C, const double* global_na,
-                    int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
-                    const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
-                    double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
-                    icikt_timings* timings, const MatrixOut* mat = nullptr) {
-  if ((!s.data && !s.csc()) || (!raw && !mat)) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  o.want_counts = counts ? 1 : 0;
-  if (!pi && o.pair_lo == 0 && o.pair_hi == tri_pairs(C) + (o.include_diag ? C : 0)) o.pair_hi = 0;  // the whole order
-  std::lock_guard<std::mutex> lock(g_cache_mu);
-  icikt_plan* p = nullptr;
-  const bool cacheable = (pi == nullptr);
-  const bool staged = want_staged(n, C, o, pi == nullptr);
-  int rc = ICIKT_OK;
-  if (cacheable && cache_matches(g_cached, n, C, o, staged) &&
-      (o.perspective != ICIKT_PERSPECTIVE_COMPLETE || g_cached->d_pw)) {
-    p = g_cached;
-    reuse_plan(p, o);
+// The plan of a call, cached in `slot` (the caller holds g_cache_mu): the slot's plan if n, C, `staged` and the
+// options that shape a plan match (device, kernel, diagonal, pair range, counts, the complete-observations buffer),
+// with the call's other options; otherwise a new plan takes the slot.
+static int cached_plan(icikt_plan*& slot, int64_t n, int64_t C, const icikt_opts& o, bool staged, icikt_plan** out) {
+  icikt_plan* p = slot;
+  if (p && p->staged == staged && p->n == n && p->C == C && p->opts.device == o.device && p->opts.kernel == o.kernel &&
+      p->opts.include_diag == o.include_diag && p->opts.pair_lo == o.pair_lo && p->opts.pair_hi == o.pair_hi &&
+      p->want_counts == (o.want_counts != 0) && (o.perspective != ICIKT_PERSPECTIVE_COMPLETE || p->d_pw)) {
+    p->opts.perspective = o.perspective;
+    p->opts.alternative = o.alternative;
+    p->opts.continuity = o.continuity;
+    p->opts.na_inf = o.na_inf;
   } else {
-    if (cacheable && g_cached) { icikt_plan_destroy(g_cached); g_cached = nullptr; }
-    rc = plan_create_impl(&p, n, C, pi, pj, P, &o, staged);
-    if (rc != ICIKT_OK) return rc;
-    if (cacheable) g_cached = p;
-  }
-  if (staged) {
-    rc = run_staged(p, s, global_na, n_global_na, mat == nullptr, raw, pvalue, taumax, completeness, status,
-                    counts, max_taumax);
-  } else {
-    rc = s.csc() ? upload_columns(p, s, 0, C) : icikt_plan_upload(p, s.data, s.ld);
-    if (rc == ICIKT_OK) rc = icikt_plan_columns(p, global_na, n_global_na);
-    if (rc == ICIKT_OK) rc = icikt_plan_pairs(p);
-  }
-  if (rc == ICIKT_OK && mat)
-    rc = icikt_plan_download_matrices(p, mat->scale_max, mat->diag_good, mat->n_good, mat->cor, raw, pvalue, taumax,
-                                      completeness, mat->status_counts, max_taumax);
-  else if (rc == ICIKT_OK && !staged)
-    rc = icikt_plan_download(p, raw, pvalue, taumax, completeness, status, counts, max_taumax);
-  if (rc == ICIKT_OK && timings) rc = icikt_plan_timings(p, timings);
-  const std::string keep = g_err;
-  if (!cacheable) {
     icikt_plan_destroy(p);
-  } else if (rc != ICIKT_OK) {
-    icikt_plan_destroy(g_cached);
-    g_cached = nullptr;
+    slot = nullptr;
+    const int rc = plan_create_impl(&p, n, C, nullptr, nullptr, 0, &o, staged);
+    *out = p;
+    if (rc != ICIKT_OK) return rc;
+    slot = p;
   }
-  if (rc != ICIKT_OK) g_err = keep;
-  return rc;
+  *out = p;
+  return ICIKT_OK;
 }
 
 int icikt_pair_from_index(int64_t C, int32_t include_diag, int64_t index, int32_t* i, int32_t* j) {
@@ -1625,64 +1578,6 @@ int icikt_measure_issue_rate(int32_t device, double* alu, double* fma, double* m
   if (fma) *fma = f;
   if (mixed) *mixed = m;
   return ICIKT_OK;
-}
-
-int icikt_all_pairs(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                    int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue,
-                    double* taumax, double* completeness, int32_t* status, int64_t* counts,
-                    double* max_taumax, icikt_timings* timings) {
-  return one_shot(dense_source(data, ld, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw, pvalue,
-                  taumax, completeness, status, counts, max_taumax, timings);
-}
-
-int icikt_all_pairs_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
-                        const double* global_na, int32_t n_global_na, const icikt_opts* opts, double* raw,
-                        double* pvalue, double* taumax, double* completeness, int32_t* status, int64_t* counts,
-                        double* max_taumax, icikt_timings* timings) {
-  const int rc = check_csc(colptr, rowidx, values, n, C);
-  if (rc != ICIKT_OK) return rc;
-  return one_shot(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, opts, raw,
-                  pvalue, taumax, completeness, status, counts, max_taumax, timings);
-}
-
-}  // extern "C"
-
-static int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                         const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts* opts, int32_t scale_max,
-                         int32_t diag_good, const int32_t* n_good, double* cor, double* raw, double* pvalue,
-                         double* taumax, double* completeness, int64_t* status_counts, double* max_taumax,
-                         icikt_timings* timings) {
-  if ((pi == nullptr) != (pj == nullptr)) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must both be given");
-  icikt_opts o;
-  if (opts) o = *opts; else icikt_default_opts(&o);
-  if (!pi && (o.pair_lo != 0 || o.pair_hi != 0))
-    return fail(ICIKT_ERR_BAD_ARG, "matrix output needs the whole pair order on one device");
-  if (!pi) o.include_diag = diag_good ? 0 : 1;  // setup_comparisons, R/kendalltau.R:191-194
-  const MatrixOut mo{scale_max, diag_good, n_good, cor, status_counts};
-  return one_shot(s, n, C, global_na, n_global_na, pi, pj, P, &o, raw, pvalue, taumax, completeness, nullptr, nullptr,
-                  max_taumax, timings, &mo);
-}
-
-extern "C" {
-
-int icikt_matrices(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                   int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts* opts,
-                   int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
-                   double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
-                   double* max_taumax, icikt_timings* timings) {
-  return matrices_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max, diag_good,
-                       n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
-}
-
-int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
-                       const double* global_na, int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
-                       const icikt_opts* opts, int32_t scale_max, int32_t diag_good, const int32_t* n_good,
-                       double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
-                       int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
-  const int rc = check_csc(colptr, rowidx, values, n, C);
-  if (rc != ICIKT_OK) return rc;
-  return matrices_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, pi, pj, P, opts, scale_max,
-                       diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
 }
 
 }  // extern "C"
@@ -2277,25 +2172,6 @@ static void topk_sides_finish(std::vector<TopkSide>& sides, int k, Held&& held, 
 
 #undef ECK
 
-// The plan of the windowed calls (cached in `slot`, see window_slots; the caller holds g_cache_mu): pair buffers of
-// one window of W pairs.
-static int window_plan(icikt_plan*& slot, int64_t n, int64_t C, int64_t W, const icikt_opts& o, icikt_plan** out) {
-  icikt_plan* p = slot;
-  if (p && p->n == n && p->C == C && p->P == W && p->opts.device == o.device && p->opts.include_diag == o.include_diag) {
-    reuse_plan(p, o);
-  } else {
-    if (p) icikt_plan_destroy(p);
-    slot = nullptr;
-    icikt_opts po = o;
-    po.pair_hi = W;  // the plan's pair buffers: one window
-    const int rc = plan_create_impl(&p, n, C, nullptr, nullptr, 0, &po, false);
-    if (rc != ICIKT_OK) return rc;
-    slot = p;
-  }
-  *out = p;
-  return ICIKT_OK;
-}
-
 extern "C" {
 
 int64_t icikt_edges_count(const icikt_edges* e) { return e ? (int64_t)e->rows.size() : 0; }
@@ -2548,10 +2424,12 @@ namespace {
 // slice and pulls the other slices of the per-column TABLES from its peers (an all-gather by peer
 // copies: K1 is not replicated and the raw matrix never travels between devices); otherwise every
 // device uploads the whole matrix and preprocesses all columns.  A cross call's job holds [X | Y]: src is X, y is Y
-// (placed from column src.C on), C = Cx + Cy, and the slices cover pairs [first, first + ptot) of the cross order.
+// (placed from column src.C on), C = Cx + Cy, and the slices cover pairs [first, first + ptot) of the cross order.  A
+// pair-list job (one worker) computes the ptot pairs (pi[k], pj[k]).
 struct MultiJob {
   ColumnSource src;
   const ColumnSource* y = nullptr;
+  const int32_t *pi = nullptr, *pj = nullptr;
   int64_t n, C;
   const double* global_na;
   int32_t n_global_na;
@@ -2567,6 +2445,7 @@ struct MultiJob {
   int device_of(int k) const { return devices ? devices[k] : k; }
   int64_t pair_lo(int k) const { return first + ptot * k / n_devices; }  // slices differ by at most one pair
   int64_t col_lo(int k) const { return C * k / n_devices; }
+  bool idle(int k) const { return n_devices > 1 && pair_lo(k + 1) <= pair_lo(k); }  // one of several, without pairs
 };
 
 void multi_probe_peers(MultiJob& J) {
@@ -2598,12 +2477,11 @@ int enable_peers(const MultiJob& J, int k) {
 }
 
 // The column phase of worker k on its plan p (rc: how getting the plan went): sharded K1 and the peer gather of the
-// tables in gather mode, otherwise the upload and K1 of all columns (skipped when the worker has no pairs).  In
+// tables in gather mode, otherwise the upload and K1 of all columns (skipped by an idle worker).  In
 // gather mode every worker passes both barriers whatever happened to it, so nobody is left waiting.  A cross job's
 // columns are those of [X | Y]: a shard that straddles column Cx uploads X's part, then Y's (upload_span).
 int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
-  const int64_t cnt = J.pair_lo(k + 1) - J.pair_lo(k);
-  if (!J.gather) return cnt <= 0 || rc != ICIKT_OK ? rc : window_columns(p, J.src, J.global_na, J.n_global_na, J.y);
+  if (!J.gather) return J.idle(k) || rc != ICIKT_OK ? rc : window_columns(p, J.src, J.global_na, J.n_global_na, J.y);
   int x_launches = 0;
   if (rc == ICIKT_OK) rc = upload_span(p, J.src, J.y, J.col_lo(k), J.col_lo(k + 1), &x_launches);
   if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
@@ -2638,30 +2516,69 @@ int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
   return rc;
 }
 
-// Worker k up to and including the pair kernel + epilogue (results stay on its device).
-int multi_worker_pairs(MultiJob& J, int k, icikt_plan** out) {
-  int rc = ICIKT_OK;
+// The cached plans of a per-pair job's workers, as window_slots: one worker takes g_cached, several one slot each.
+icikt_plan** pair_slots(const MultiJob& J) { return J.n_devices == 1 ? &g_cached : g_cached_multi; }
+
+// The per-pair and matrix calls as a job over the caller's pair range (0, 0: all pairs) or pair list, with the checks
+// of their arguments that need no device.
+int pairs_job(MultiJob& J, const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+              const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts& o, const int32_t* devices) {
+  if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
+  if (C > 2147483647LL) return fail(ICIKT_ERR_BAD_ARG, "too many columns");
+  if (!s.csc() && s.ld < n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
+  const int64_t all = tri_pairs(C) + (o.include_diag ? C : 0);
+  const int64_t lo = o.pair_lo, hi = (o.pair_lo == 0 && o.pair_hi == 0) ? all : o.pair_hi;
+  if (!pi && (lo < 0 || hi > all || lo > hi)) return fail(ICIKT_ERR_BAD_ARG, "pair_lo/pair_hi out of range");
+  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.pi = pi; J.pj = pj; J.devices = devices; J.base = o;
+  J.first = pi ? 0 : lo;
+  J.ptot = pi ? P : hi - lo;
+  return ICIKT_OK;
+}
+
+// A lone worker over the whole pair order of a large input runs the pipelined call (run_staged).
+bool job_staged(const MultiJob& J) {
+  return J.n_devices == 1 && !J.pi && J.first == 0 && J.ptot == tri_pairs(J.C) + (J.base.include_diag ? J.C : 0) &&
+         want_staged(J.n, J.C, J.base);
+}
+
+// the per-pair output arrays of a call, indexed from 0 = the job's first pair
+struct PairArrays {
+  double *raw, *pvalue, *taumax, *completeness;
+  int32_t* status;
+  int64_t* counts;
+};
+
+// Worker k of a per-pair job: its plan (slots[k]; a pair list's is built from J.pi / J.pj), the column phase and the
+// pair kernel + epilogue, then, given `to`, the download of its slice at its offset from J.first (mx: the slice's
+// maximum taumax); without `to` the results stay on its device.  `staged` (job_staged): all of it as the pipelined
+// call.  An idle worker only takes part in the column phase.
+int pairs_worker(MultiJob& J, int k, icikt_plan** slots, bool staged, const PairArrays* to, icikt_plan** out,
+                 double* mx) {
   icikt_opts o = J.base;
   o.device = J.device_of(k);
-  o.pair_lo = J.pair_lo(k);
-  o.pair_hi = J.pair_lo(k + 1);
-  const int64_t cnt = o.pair_hi - o.pair_lo;
-  // one cached plan per slot, like the one-shot entry points: repeated calls of the same shape do not
-  // pay the device allocations again
-  icikt_plan*& slot = g_cached_multi[k];
-  icikt_plan* p = nullptr;
-  if (cache_matches(slot, J.n, J.C, o, false) && (o.perspective != ICIKT_PERSPECTIVE_COMPLETE || slot->d_pw)) {
-    p = slot;
-    reuse_plan(p, o);
+  o.pair_lo = staged ? 0 : J.pair_lo(k);  // a staged plan covers the whole order as 0, 0
+  o.pair_hi = staged ? 0 : J.pair_lo(k + 1);
+  int rc;
+  if (J.pi) {
+    rc = plan_create_impl(out, J.n, J.C, J.pi, J.pj, J.ptot, &o, false);
+    slots[k] = *out;
   } else {
-    if (slot) { icikt_plan_destroy(slot); slot = nullptr; }
-    rc = icikt_plan_create(&p, J.n, J.C, nullptr, nullptr, 0, &o);
-    if (rc == ICIKT_OK) slot = p;
+    rc = cached_plan(slots[k], J.n, J.C, o, staged, out);
   }
-  *out = p;
+  icikt_plan* p = *out;
+  if (staged) {
+    const PairArrays d = to ? *to : PairArrays{};
+    return rc != ICIKT_OK ? rc : run_staged(p, J.src, J.global_na, J.n_global_na, to != nullptr, d.raw, d.pvalue,
+                                            d.taumax, d.completeness, d.status, d.counts, mx);
+  }
   rc = multi_worker_columns(J, k, p, rc);
-  if (rc == ICIKT_OK && cnt > 0) rc = icikt_plan_pairs(p);
-  return rc;
+  if (rc == ICIKT_OK && !J.idle(k)) rc = icikt_plan_pairs(p);
+  if (rc != ICIKT_OK || J.idle(k) || !to) return rc;
+  const int64_t off = J.pair_lo(k) - J.first;
+  auto at = [off](auto* a, int64_t per_pair = 1) { return a ? a + off * per_pair : a; };
+  return icikt_plan_download(p, at(to->raw), at(to->pvalue), at(to->taumax), at(to->completeness), at(to->status),
+                             at(to->counts, ICIKT_NCOUNTS), mx);
 }
 
 struct MultiWork {
@@ -2717,72 +2634,68 @@ int run_workers(const MultiJob& J, icikt_plan** slots, std::vector<MultiWork>& w
   return multi_collect(work, max_taumax, timings);
 }
 
-int all_pairs_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                         const icikt_opts* opts, const int32_t* devices, int32_t n_devices, double* raw,
-                         double* pvalue, double* taumax, double* completeness, int32_t* status, int64_t* counts,
-                         double* max_taumax, icikt_timings* timings) {
-  if ((!s.data && !s.csc()) || !raw) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
+// The per-pair calls: icikt_all_pairs and icikt_pair_list are the job of one worker on opts->device, the _multi twins
+// that of the caller's devices.
+int pairs_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+               const int32_t* pi, const int32_t* pj, int64_t P, icikt_opts o, const int32_t* devices, int32_t n_devices,
+               const PairArrays& to, double* max_taumax, icikt_timings* timings) {
+  if ((!s.data && !s.csc()) || !to.raw) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
   if (n_devices < 1 || n_devices > 64) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..64");
-  if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
-  if (!s.csc() && s.ld < n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
+  o.want_counts = to.counts ? 1 : 0;
   MultiJob J(n_devices);
-  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices;
-  if (opts) J.base = *opts; else icikt_default_opts(&J.base);
-  J.base.want_counts = counts ? 1 : 0;
-  J.ptot = tri_pairs(C) + (J.base.include_diag ? C : 0);
+  int rc = pairs_job(J, s, n, C, global_na, n_global_na, pi, pj, P, o, devices);
+  if (rc != ICIKT_OK) return rc;
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
   multi_probe_peers(J);
+  const bool staged = job_staged(J);
+  icikt_plan* list_plan = nullptr;  // a pair list's plan is freed at the end of the call
+  icikt_plan** slots = pi ? &list_plan : pair_slots(J);
   std::vector<MultiWork> work;
-  return run_workers(J, g_cached_multi, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
+  rc = run_workers(J, slots, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
     icikt_plan* p = nullptr;
-    int rc = multi_worker_pairs(J, k, &p);
-    const int64_t lo = J.pair_lo(k), cnt = J.pair_lo(k + 1) - lo;
-    if (rc == ICIKT_OK && cnt > 0)
-      rc = icikt_plan_download(p, raw + lo, pvalue ? pvalue + lo : nullptr, taumax ? taumax + lo : nullptr,
-                               completeness ? completeness + lo : nullptr, status ? status + lo : nullptr,
-                               counts ? counts + lo * ICIKT_NCOUNTS : nullptr, &w.mx);
-    if (rc == ICIKT_OK && cnt > 0) rc = icikt_plan_timings(p, &w.tm);
-    return rc;
+    int r = pairs_worker(J, k, slots, staged, &to, &p, &w.mx);
+    if (r == ICIKT_OK && timings && !J.idle(k)) r = icikt_plan_timings(p, &w.tm);
+    return r;
   });
+  icikt_plan_destroy(list_plan);
+  return rc;
 }
 
-int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
-                        const icikt_opts* opts, const int32_t* devices, int32_t n_devices, int32_t scale_max,
-                        int32_t diag_good, const int32_t* n_good, double* cor, double* raw, double* pvalue,
-                        double* taumax, double* completeness, int64_t* status_counts, double* max_taumax,
-                        icikt_timings* timings) {
-  if (!s.data && !s.csc()) return fail(ICIKT_ERR_BAD_ARG, "data must not be NULL");
-  if (n_devices < 1 || n_devices > kMaxMatrixDevices) return fail(ICIKT_ERR_BAD_ARG, "n_devices must be 1..16");
-  if (n < 1 || C < 1) return fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1");
-  icikt_opts base;
-  if (opts) base = *opts; else icikt_default_opts(&base);
-  base.include_diag = diag_good ? 0 : 1;  // setup_comparisons, R/kendalltau.R:191-194
-  base.pair_lo = base.pair_hi = 0;
-  const int64_t ptot = tri_pairs(C) + (base.include_diag ? C : 0);
+// The matrix calls: one worker computes its pairs and fills the matrices (icikt_plan_download_matrices); several, with
+// peer access between them, fill a block of columns each from every device's results (matrix_block_fill_kernel).
+int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_na, int32_t n_global_na,
+                  const int32_t* pi, const int32_t* pj, int64_t P, icikt_opts o, const int32_t* devices,
+                  int32_t n_devices, int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor,
+                  double* raw, double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
+                  double* max_taumax, icikt_timings* timings) {
+  if (!pi) o.include_diag = diag_good ? 0 : 1;  // setup_comparisons, R/kendalltau.R:191-194
+  o.want_counts = 0;
   MultiJob J(n_devices);
-  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = base; J.base.want_counts = 0; J.ptot = ptot;
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);
-    multi_probe_peers(J);
-  }
-  if (n_devices == 1 || !J.peers_ok || ptot < n_devices || C < n_devices) {
-    // one device, or devices that cannot read each other's results: the single-device path
-    base.device = J.device_of(0);
-    return matrices_impl(s, n, C, global_na, n_global_na, nullptr, nullptr, 0, &base, scale_max, diag_good, n_good,
-                         cor, raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
-  }
-  if (!s.csc() && s.ld < n) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
+  int rc = pairs_job(J, s, n, C, global_na, n_global_na, pi, pj, P, o, devices);
+  if (rc != ICIKT_OK) return rc;
   std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+  multi_probe_peers(J);
+  // devices that cannot read each other's results, or fewer pairs or columns than devices: one worker on devices[0]
+  if (!J.peers_ok || J.ptot < J.n_devices || C < J.n_devices) J.n_devices = 1;
+  const bool staged = job_staged(J);
+  icikt_plan* list_plan = nullptr;  // a pair list's plan is freed at the end of the call
+  icikt_plan** slots = pi ? &list_plan : pair_slots(J);
+  const int n_dev = J.n_devices;
   double* outs[5] = {cor, raw, pvalue, taumax, completeness};
   std::vector<MultiWork> work;
   std::vector<int32_t> good((size_t)C, 0);
   if (n_good) std::copy(n_good, n_good + C, good.begin());
-  std::vector<icikt_plan*> plans((size_t)n_devices, nullptr);
-  const int rc = run_workers(J, g_cached_multi, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
+  std::vector<icikt_plan*> plans((size_t)n_dev, nullptr);
+  rc = run_workers(J, slots, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
     icikt_plan* p = nullptr;
-    w.rc = multi_worker_pairs(J, k, &p);
+    w.rc = pairs_worker(J, k, slots, staged, nullptr, &p, nullptr);
+    if (n_dev == 1) {  // the whole matrices from this worker's results
+      if (w.rc == ICIKT_OK)
+        w.rc = icikt_plan_download_matrices(p, scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness,
+                                            status_counts, &w.mx);
+      if (w.rc == ICIKT_OK && timings) w.rc = icikt_plan_timings(p, &w.tm);
+      return w.rc;
+    }
     unsigned long long bits = 0;
     if (w.rc == ICIKT_OK) {
       if (cudaMemcpyAsync(&bits, p->d_maxbits, sizeof(bits), cudaMemcpyDeviceToHost, p->stream) != cudaSuccess ||
@@ -2798,7 +2711,7 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
     J.barrier.wait();  // every slice of the pair results is complete on its device
     bool all_ok = true;
     double mx = std::nan("");
-    for (int j = 0; j < n_devices; ++j) {
+    for (int j = 0; j < n_dev; ++j) {
       all_ok = all_ok && plans[(size_t)j] != nullptr;
       if (work[(size_t)j].mx == work[(size_t)j].mx && !(mx >= work[(size_t)j].mx)) mx = work[(size_t)j].mx;
     }
@@ -2827,14 +2740,14 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
       CK(cudaEventRecord(p->ev[6], p->stream));
       CK(cudaMemsetAsync(p->d_hist, 0, 16 * sizeof(unsigned long long), p->stream));
       BlockFill f{};
-      f.n_dev = n_devices;
-      for (int j = 0; j < n_devices; ++j) {
+      f.n_dev = n_dev;
+      for (int j = 0; j < n_dev; ++j) {
         const icikt_plan* q = plans[(size_t)j];
         f.tau[j] = q->d_tau; f.pvalue[j] = q->d_p; f.taumax[j] = q->d_tm; f.completeness[j] = q->d_comp;
         f.status[j] = q->d_status;
         f.pair_lo[j] = J.pair_lo(j);
       }
-      f.pair_lo[n_devices] = ptot;
+      f.pair_lo[n_dev] = J.ptot;
       f.n = n; f.C = C; f.c_lo = c_lo; f.c_hi = c_hi;
       f.scale_max = scale_max != 0; f.diag_good = diag_good != 0;
       f.max_taumax = mx;
@@ -2862,7 +2775,8 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
     J.barrier.wait();  // nobody's results are freed before every block has been filled
     return w.rc;
   });
-  if (rc != ICIKT_OK) return rc;
+  icikt_plan_destroy(list_plan);
+  if (rc != ICIKT_OK || n_dev == 1) return rc;
   if (status_counts) {
     int64_t bad = 0;
     for (int q = 1; q < ICIKT_NSTATUS; ++q) {
@@ -2870,7 +2784,7 @@ int matrices_multi_impl(const ColumnSource& s, int64_t n, int64_t C, const doubl
       for (const MultiWork& w : work) status_counts[q] += (int64_t)w.hist[q];
       bad += status_counts[q];
     }
-    status_counts[0] = ptot - bad;
+    status_counts[0] = J.ptot - bad;
   }
   return ICIKT_OK;
 }
@@ -2899,12 +2813,10 @@ icikt_plan** window_slots(const MultiJob& J) { return J.n_devices == 1 ? &g_cach
 int window_multi_worker(MultiJob& J, int k, icikt_plan** out) {
   icikt_opts o = J.base;
   o.device = J.device_of(k);
-  const int64_t W = std::max<int64_t>(1, std::min(edge_window(), J.pair_lo(k + 1) - J.pair_lo(k)));
-  icikt_plan* p = nullptr;
-  int rc = window_plan(window_slots(J)[k], J.n, J.C, W, o, &p);
-  *out = p;
-  rc = multi_worker_columns(J, k, p, rc);
-  if (rc == ICIKT_OK) CK(cudaSetDevice(p->device));
+  o.pair_hi = std::max<int64_t>(1, std::min(edge_window(), J.pair_lo(k + 1) - J.pair_lo(k)));  // pair_lo is 0
+  int rc = cached_plan(window_slots(J)[k], J.n, J.C, o, false, out);
+  rc = multi_worker_columns(J, k, *out, rc);
+  if (rc == ICIKT_OK) CK(cudaSetDevice((*out)->device));
   return rc;
 }
 
@@ -3427,13 +3339,41 @@ int cross_edges_padj_impl(const icikt_input* x, const icikt_input* y, int64_t n,
 
 extern "C" {
 
+int icikt_all_pairs(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                    int32_t n_global_na, const icikt_opts* opts, double* raw, double* pvalue,
+                    double* taumax, double* completeness, int32_t* status, int64_t* counts,
+                    double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return pairs_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, o, &o.device, 1,
+                    PairArrays{raw, pvalue, taumax, completeness, status, counts}, max_taumax, timings);
+}
+
+int icikt_all_pairs_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                        const double* global_na, int32_t n_global_na, const icikt_opts* opts, double* raw,
+                        double* pvalue, double* taumax, double* completeness, int32_t* status, int64_t* counts,
+                        double* max_taumax, icikt_timings* timings) {
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  const icikt_opts o = opts_or_default(opts);
+  return pairs_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, o,
+                    &o.device, 1, PairArrays{raw, pvalue, taumax, completeness, status, counts}, max_taumax, timings);
+}
+
+// the options of a _multi call: opts->device, pair_lo and pair_hi are ignored
+static icikt_opts multi_opts(const icikt_opts* opts) {
+  icikt_opts o = opts_or_default(opts);
+  o.pair_lo = o.pair_hi = 0;
+  return o;
+}
+
 int icikt_all_pairs_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
                           int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
                           int32_t n_devices, double* raw, double* pvalue, double* taumax,
                           double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
                           icikt_timings* timings) {
-  return all_pairs_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, raw,
-                              pvalue, taumax, completeness, status, counts, max_taumax, timings);
+  return pairs_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, nullptr, nullptr, 0, multi_opts(opts),
+                    devices, n_devices, PairArrays{raw, pvalue, taumax, completeness, status, counts}, max_taumax,
+                    timings);
 }
 
 int icikt_all_pairs_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n,
@@ -3443,8 +3383,75 @@ int icikt_all_pairs_multi_csc(const int64_t* colptr, const int32_t* rowidx, cons
                               icikt_timings* timings) {
   const int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return all_pairs_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices,
-                              n_devices, raw, pvalue, taumax, completeness, status, counts, max_taumax, timings);
+  return pairs_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, nullptr, nullptr, 0,
+                    multi_opts(opts), devices, n_devices, PairArrays{raw, pvalue, taumax, completeness, status, counts},
+                    max_taumax, timings);
+}
+
+int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                    int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
+                    const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
+                    double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
+                    icikt_timings* timings) {
+  if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
+  const icikt_opts o = opts_or_default(opts);
+  return pairs_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, pi, pj, P, o, &o.device, 1,
+                    PairArrays{raw, pvalue, taumax, completeness, status, counts}, max_taumax, timings);
+}
+
+int icikt_pair_list_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                        const double* global_na, int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
+                        const icikt_opts* opts, double* raw, double* pvalue, double* taumax, double* completeness,
+                        int32_t* status, int64_t* counts, double* max_taumax, icikt_timings* timings) {
+  if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
+  const int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  const icikt_opts o = opts_or_default(opts);
+  return pairs_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, pi, pj, P, o, &o.device, 1,
+                    PairArrays{raw, pvalue, taumax, completeness, status, counts}, max_taumax, timings);
+}
+
+// the checks icikt_matrices[_csc] make first
+static int check_matrices_one(const ColumnSource& s, const int32_t* pi, const int32_t* pj, const icikt_opts& o) {
+  if ((pi == nullptr) != (pj == nullptr)) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must both be given");
+  if (!pi && (o.pair_lo != 0 || o.pair_hi != 0))
+    return fail(ICIKT_ERR_BAD_ARG, "matrix output needs the whole pair order on one device");
+  if (!s.data && !s.csc()) return fail(ICIKT_ERR_BAD_ARG, "data and raw must not be NULL");
+  return ICIKT_OK;
+}
+
+// ... and icikt_matrices_multi[_csc]
+static int check_matrices_multi(const ColumnSource& s, int32_t n_devices) {
+  if (!s.data && !s.csc()) return fail(ICIKT_ERR_BAD_ARG, "data must not be NULL");
+  return check_window_devices(n_devices);
+}
+
+int icikt_matrices(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
+                   int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P, const icikt_opts* opts,
+                   int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
+                   double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
+                   double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  const ColumnSource s = dense_source(data, ld, C);
+  const int rc = check_matrices_one(s, pi, pj, o);
+  if (rc != ICIKT_OK) return rc;
+  return matrices_impl(s, n, C, global_na, n_global_na, pi, pj, P, o, &o.device, 1, scale_max, diag_good, n_good, cor,
+                       raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
+}
+
+int icikt_matrices_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
+                       const double* global_na, int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
+                       const icikt_opts* opts, int32_t scale_max, int32_t diag_good, const int32_t* n_good,
+                       double* cor, double* raw, double* pvalue, double* taumax, double* completeness,
+                       int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  int rc = check_csc(colptr, rowidx, values, n, C);
+  if (rc != ICIKT_OK) return rc;
+  const icikt_opts o = opts_or_default(opts);
+  const ColumnSource s = csc_source(colptr, rowidx, values, C);
+  rc = check_matrices_one(s, pi, pj, o);
+  if (rc != ICIKT_OK) return rc;
+  return matrices_impl(s, n, C, global_na, n_global_na, pi, pj, P, o, &o.device, 1, scale_max, diag_good, n_good, cor,
+                       raw, pvalue, taumax, completeness, status_counts, max_taumax, timings);
 }
 
 int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
@@ -3452,9 +3459,12 @@ int icikt_matrices_multi(const double* data, int64_t n, int64_t C, int64_t ld, c
                          int32_t scale_max, int32_t diag_good, const int32_t* n_good, double* cor, double* raw,
                          double* pvalue, double* taumax, double* completeness, int64_t* status_counts,
                          double* max_taumax, icikt_timings* timings) {
-  return matrices_multi_impl(dense_source(data, ld, C), n, C, global_na, n_global_na, opts, devices, n_devices, scale_max,
-                             diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax,
-                             timings);
+  const ColumnSource s = dense_source(data, ld, C);
+  const int rc = check_matrices_multi(s, n_devices);
+  if (rc != ICIKT_OK) return rc;
+  return matrices_impl(s, n, C, global_na, n_global_na, nullptr, nullptr, 0, multi_opts(opts), devices, n_devices,
+                       scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax,
+                       timings);
 }
 
 int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
@@ -3463,11 +3473,14 @@ int icikt_matrices_multi_csc(const int64_t* colptr, const int32_t* rowidx, const
                              const int32_t* n_good, double* cor, double* raw, double* pvalue, double* taumax,
                              double* completeness, int64_t* status_counts, double* max_taumax,
                              icikt_timings* timings) {
-  const int rc = check_csc(colptr, rowidx, values, n, C);
+  int rc = check_csc(colptr, rowidx, values, n, C);
   if (rc != ICIKT_OK) return rc;
-  return matrices_multi_impl(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, opts, devices,
-                             n_devices, scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness,
-                             status_counts, max_taumax, timings);
+  const ColumnSource s = csc_source(colptr, rowidx, values, C);
+  rc = check_matrices_multi(s, n_devices);
+  if (rc != ICIKT_OK) return rc;
+  return matrices_impl(s, n, C, global_na, n_global_na, nullptr, nullptr, 0, multi_opts(opts), devices, n_devices,
+                       scale_max, diag_good, n_good, cor, raw, pvalue, taumax, completeness, status_counts, max_taumax,
+                       timings);
 }
 
 int icikt_all_pairs_edges(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
@@ -3598,27 +3611,6 @@ int icikt_cross_topk_multi(const icikt_input* x, const icikt_input* y, int64_t n
                            const icikt_topk_lists* y_side, double* max_taumax, icikt_timings* timings) {
   return cross_topk_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, k, by, scale_max,
                          x_side, y_side, max_taumax, timings);
-}
-
-int icikt_pair_list(const double* data, int64_t n, int64_t C, int64_t ld, const double* global_na,
-                    int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
-                    const icikt_opts* opts, double* raw, double* pvalue, double* taumax,
-                    double* completeness, int32_t* status, int64_t* counts, double* max_taumax,
-                    icikt_timings* timings) {
-  if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
-  return one_shot(dense_source(data, ld, C), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue, taumax,
-                  completeness, status, counts, max_taumax, timings);
-}
-
-int icikt_pair_list_csc(const int64_t* colptr, const int32_t* rowidx, const double* values, int64_t n, int64_t C,
-                        const double* global_na, int32_t n_global_na, const int32_t* pi, const int32_t* pj, int64_t P,
-                        const icikt_opts* opts, double* raw, double* pvalue, double* taumax, double* completeness,
-                        int32_t* status, int64_t* counts, double* max_taumax, icikt_timings* timings) {
-  if (!pi || !pj) return fail(ICIKT_ERR_BAD_ARG, "pi and pj must not be NULL");
-  const int rc = check_csc(colptr, rowidx, values, n, C);
-  if (rc != ICIKT_OK) return rc;
-  return one_shot(csc_source(colptr, rowidx, values, C), n, C, global_na, n_global_na, pi, pj, P, opts, raw, pvalue,
-                  taumax, completeness, status, counts, max_taumax, timings);
 }
 
 int icikt_pnorm_device(const double* z, int64_t n, int32_t lower_tail, double* out, int32_t device) {

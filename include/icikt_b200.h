@@ -139,7 +139,8 @@ int icikt_all_pairs(const double* data, int64_t n, int64_t C, int64_t ld,
  * (SURVEY.md 8e).  devices == NULL means ordinals 0..n_devices-1; opts->device, pair_lo and
  * pair_hi are ignored.  timings (may be NULL) receives the slowest device's figures.
  * With n_devices == 1 the work runs on the calling thread, whose current CUDA device is devices[0]
- * afterwards, as after every single-device call.                                               */
+ * afterwards, as after every single-device call, and it is icikt_all_pairs' work: a large input takes
+ * the pipelined path (icikt_stage_table), with the timings described above icikt_timings.      */
 int icikt_all_pairs_multi(const double* data, int64_t n, int64_t C, int64_t ld,
                           const double* global_na, int32_t n_global_na, const icikt_opts* opts,
                           const int32_t* devices, int32_t n_devices, double* raw, double* pvalue,

@@ -984,6 +984,9 @@ def test_pipelined_one_shot_matches_plain_call(monkeypatch, persp, diag, kind):
     piped = ik.run_pairs(x, (), **kw)
     _same_pairs(piped, plain, f"pipelined {persp}")
     assert piped["timings"]["n_launches"] > plain["timings"]["n_launches"], "the pipelined path did not run"
+    one = ik.run_pairs(x, (), devices=[0], **kw)  # icikt_all_pairs_multi with one device: the same pipelined call
+    _same_pairs(one, plain, f"pipelined, devices=[0] {persp}")
+    assert one["timings"]["n_launches"] == piped["timings"]["n_launches"], "devices=[0] did not take the pipelined path"
     again = ik.run_pairs(x, (), **kw)  # the cached staged plan, second use
     _same_pairs(again, plain, f"pipelined, cached plan {persp}")
     xp = torch.from_numpy(np.asfortranarray(x).T.copy()).pin_memory().numpy().T  # pinned, column-major

@@ -215,8 +215,8 @@ def test_max_edges_without_scale_max():
 
 
 def test_interleaved_calls_keep_their_results():
-    """the multi-device window plans, the single-device window plan and the per-pair multi plans do not disturb each
-    other"""
+    """the multi-device window plans, the single-device window plan, the per-pair multi plans and the per-pair plan of
+    one device (the single-device call and devices=[0], alternated) do not disturb each other"""
     x = gen(1500, 90, "mixed", 0.1, seed=71)
     devices = DEVICE_LISTS[-1]
     e0 = ik.run_edges(x, (), min_abs_cor=0.3, devices=devices)
@@ -224,7 +224,12 @@ def test_interleaved_calls_keep_their_results():
     s0 = ik.run_edges(x, (), min_abs_cor=0.3)
     p0 = ik.run_pairs(x, (), devices=devices)
     m0 = _lib.run_matrices(x, (), devices=devices)
+    s1 = ik.run_pairs(x, ())
     for _ in range(2):
+        for one in ([0], None):
+            p = ik.run_pairs(x, (), devices=one)
+            for key in ("raw", "pvalue", "taumax", "completeness", "status"):
+                assert np.array_equal(p[key].view(np.uint8), s1[key].view(np.uint8)), (one, key)
         E.same(ik.run_edges(x, (), min_abs_cor=0.3, devices=devices), e0, "multi edges again")
         T.same(ik.run_topk(x, (), k=6, devices=devices), k0, "multi top-k again")
         E.same(ik.run_edges(x, (), min_abs_cor=0.3), s0, "single edges again")

@@ -14,8 +14,13 @@ field, and a hash of every output array.  Every output must be bit-identical bet
 median must lie within the other build's spread.  The card's name, power limit and max SM clock come from the same
 run.
 
-    python tools/window_ab.py --lib-a OLD.so --lib-b NEW.so [--reps 2] [--steps 3] [--sizes big,small] [--only TEXT]
-                              [--out f.json]
+--calls pairs runs the per-pair and matrix calls instead: run_pairs over all pairs at the benchmark's target (the
+pipelined call on one GPU; 200 x 50 at the small size), run_pairs with a list of 10^5 random pairs of that matrix (500
+at the small size, one GPU only), and run_matrices (diag_good) at 2 000 x 5 000 (200 x 50), each dense and CSC, on one
+GPU and, where the call takes devices, on devices = [0, 0].
+
+    python tools/window_ab.py --lib-a OLD.so --lib-b NEW.so [--calls windowed|pairs] [--reps 2] [--steps 3]
+                              [--sizes big,small] [--only TEXT] [--out f.json]
 
 --only keeps the cases whose name contains TEXT (e.g. "cross big": the per-pair cross call at the large size).
 """
@@ -92,11 +97,45 @@ def cases(sizes):
                                                                                           side="both", devices=v)
 
 
+def pair_cases(sizes):
+    """(name, call) for the per-pair and matrix calls: run_pairs over all pairs (at the benchmark's target, the
+    pipelined call on one GPU), run_pairs with a pair list, and run_matrices (all pairs, diag_good)"""
+    import scipy.sparse as sp
+    from icikendalltau_b200 import _lib, synth
+
+    def forms(a):
+        return {"dense": a, "csc": sp.csc_matrix(np.nan_to_num(a, nan=0.0))}
+
+    arms = (("one_gpu", None), ("devices_0_0", [0, 0]))
+    for size in sizes:
+        if size == "big":
+            x, _ = synth.make("target")
+            P, (mn, mc) = 100_000, (2000, 5000)
+        else:
+            x = synth.left_censored(200, 50, 0.20, seed=synth.SEEDS["config5"])
+            P, (mn, mc) = 500, (200, 50)
+        n, C = x.shape
+        rng = np.random.default_rng(5)
+        pi, pj = rng.integers(0, C, P).astype(np.int32), rng.integers(0, C, P).astype(np.int32)
+        for form, data in forms(x).items():
+            tag = f"{size} {n}x{C} {form}"
+            yield f"pair_list {tag} P={P} one_gpu", lambda d=data: _lib.run_pairs(d, GLOBAL_NA, pi=pi, pj=pj)
+            for arm, dev in arms:
+                yield f"pairs {tag} {arm}", lambda d=data, v=dev: _lib.run_pairs(d, GLOBAL_NA, devices=v)
+        del x, data
+        m = synth.left_censored(mn, mc, 0.20, seed=synth.SEEDS["config5"])
+        for form, data in forms(m).items():
+            for arm, dev in arms:
+                yield f"matrices {size} {mn}x{mc} {form} {arm}", lambda d=data, v=dev: _lib.run_matrices(d, GLOBAL_NA,
+                                                                                                        devices=v)
+
+
 def worker(a):
     """one process, one build: every case once for warm-up, then its timed calls; one JSON document on stdout"""
     sys.path.insert(0, ROOT)
     res = {}
-    for name, call in cases(a.sizes.split(",")):
+    sizes = a.sizes.split(",")
+    for name, call in (pair_cases(sizes) if a.calls == "pairs" else cases(sizes)):
         if a.only not in name:
             continue
         call()
@@ -121,20 +160,22 @@ def main():
     ap.add_argument("--small-steps", type=int, default=30)
     ap.add_argument("--sizes", default="big,small")
     ap.add_argument("--only", default="")
+    ap.add_argument("--calls", choices=("windowed", "pairs"), default="windowed")
     ap.add_argument("--out", default=None)
     ap.add_argument("--worker", action="store_true")
     a = ap.parse_args()
     if a.worker:
         return worker(a)
     libs = {"a": os.path.abspath(a.lib_a), "b": os.path.abspath(a.lib_b)}
-    res = dict(card=card(), libs=libs, reps=a.reps, steps=a.steps, small_steps=a.small_steps, only=a.only, cases={})
+    res = dict(card=card(), libs=libs, reps=a.reps, steps=a.steps, small_steps=a.small_steps, only=a.only,
+               calls=a.calls, cases={})
     print(json.dumps(res["card"]), flush=True)
     runs = {"a": [], "b": []}
     for rep in range(a.reps):
         for arm in ("a", "b") if rep % 2 == 0 else ("b", "a"):
             t0 = time.perf_counter()
             cmd = [sys.executable, os.path.abspath(__file__), "--worker", "--steps", str(a.steps),
-                   "--small-steps", str(a.small_steps), "--sizes", a.sizes, "--only", a.only]
+                   "--small-steps", str(a.small_steps), "--sizes", a.sizes, "--only", a.only, "--calls", a.calls]
             out = subprocess.run(cmd, env=dict(os.environ, ICIKT_LIB_PATH=libs[arm]), capture_output=True, text=True)
             if out.returncode:
                 sys.stderr.write(out.stderr)
