@@ -357,6 +357,10 @@ def run_pairs(data, global_na=(), pi=None, pj=None, want_counts=False, devices=N
     devices: list of CUDA ordinals -> icikt_all_pairs_multi (all pairs only): every device takes a
     contiguous slice of the pair order.
     """
+    if devices is not None and (opt_kw.get("pair_lo", 0) or opt_kw.get("pair_hi", 0)):
+        # icikt_all_pairs_multi ignores the slice and writes every pair: buffers sized for the slice would overflow
+        raise ValueError("pair_lo / pair_hi select a slice on one device: over several devices run_pairs covers "
+                         "all pairs")
     L = load()
     lead, sfx, n, C, keep_alive = _matrix_args(data)
     o = make_opts(want_counts=want_counts, **opt_kw)
