@@ -23,6 +23,7 @@
 #include "icikt_cross.cuh"
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
+#include "icikt_owned.h"
 #include "icikt_padj.cuh"
 #include "icikt_topk.cuh"
 
@@ -55,9 +56,21 @@ int launch_fail(const char* what) {
     if (e_ != cudaSuccess) return cuda_fail(e_, #call);  \
   } while (0)
 
+// CK for the calls that allocate: running out of memory is ICIKT_ERR_ALLOC
+#define ECK(call)                                                                                              \
+  do {                                                                                                         \
+    cudaError_t e_ = (call);                                                                                   \
+    if (e_ != cudaSuccess)                                                                                     \
+      return e_ == cudaErrorMemoryAllocation ? (cudaGetLastError(), fail(ICIKT_ERR_ALLOC, "allocation failed: " #call)) \
+                                             : cuda_fail(e_, #call);                                           \
+  } while (0)
+
+// room for `count` elements in `a`, and `view` (a table the kernels take as a plain pointer) on it
 template <typename T>
-cudaError_t dmalloc(T** p, size_t count) {
-  return cudaMalloc(reinterpret_cast<void**>(p), std::max<size_t>(count, 1) * sizeof(T));
+cudaError_t reserve_view(DeviceArray<T>& a, T*& view, size_t count) {
+  const cudaError_t e = a.reserve(count);
+  view = a.get();
+  return e;
 }
 
 int64_t tri_pairs(int64_t C) { return C * (C - 1) / 2; }
@@ -183,62 +196,69 @@ void build_stage_table(int64_t C, bool include_diag, int64_t cta_slots, int n_bl
 struct icikt_plan {
   int device = 0;
   int n_sm = 0;
-  cudaStream_t stream = nullptr;
+  // the streams come before every buffer and event, so that those are released first
+  Stream stream;
+  Stream copy_stream;  // uploads and downloads of a staged run and of the window walk
   int64_t n = 0, C = 0, P = 0;
   icikt_opts opts{};
   bool want_counts = false;
 
-  double* d_data_own = nullptr;
+  DeviceArray<double> d_data_own;
   const double* d_data = nullptr;
   int64_t ld = 0;
-  double* d_global_na = nullptr;
+  DeviceArray<double> d_global_na;
   // CSC input (the *_csc entry points): the stored entries on the device, each at its global entry number;
   // csc_expand_kernel rebuilds d_data_own from them ahead of K1.  Kept with the plan, grown on demand.
-  int64_t* d_colptr = nullptr;  // [C + 1]
-  int32_t* d_rowidx = nullptr;
-  double* d_values = nullptr;
-  int64_t csc_cap = 0;                   // entries d_rowidx / d_values hold
+  DeviceArray<int64_t> d_colptr;  // [C + 1]
+  DeviceArray<int32_t> d_rowidx;
+  DeviceArray<double> d_values;
   int64_t expand_lo = 0, expand_hi = 0;  // columns uploaded as CSC and not expanded yet
   int64_t expand_dst = 0;                // ... and the matrix column their column 0 lands on (cross calls: Y at Cx)
 
+  // the column tables and the column path's scratch as the kernels take them, and the memory behind them
   ColumnTables tab;
   ColumnWork wk;
+  struct {
+    DeviceArray<uint16_t> perm, rank, trow, trun, tend, lgrp, gstart, vals_in;
+    DeviceArray<uint32_t> tord, nabits, firstbits, gpos;
+    DeviceArray<ColStats> stats;
+    DeviceArray<int32_t> max_tied;
+    DeviceArray<unsigned long long> keys_in, keys_out;
+  } col_mem;
   bool columns_done = false;
   // launch shapes of the pair kernel, one per tier (see tiled_shape): no large tie groups /
   // large tie groups sorted in place / pass B.  All are enqueued; the device-side maxima over the
   // columns pick the one that runs (no host round trip).
   TiledShape shape, shape_mid, shape_heavy;
-  unsigned char* d_scratch = nullptr;  // global-memory variant of the pair kernel
-  size_t scratch_bytes = 0;
+  DeviceArray<unsigned char> d_scratch;  // global-memory variant of the pair kernel
 
   std::vector<PairUnit> units;
   int max_unit_pairs = 1;  // longest unit
-  PairUnit* d_units = nullptr;
-  int32_t* d_pj = nullptr;
-  PairRaw* d_raw = nullptr;
-  PairComplete* d_pw = nullptr;  // complete-observations mode
+  DeviceArray<PairUnit> d_units;
+  DeviceArray<int32_t> d_pj;
+  DeviceArray<PairRaw> d_raw;
+  DeviceArray<PairComplete> d_pw;  // complete-observations mode
   // results, packed in one allocation so that one copy brings them to the host:
   // [tau P][pvalue P][taumax P][completeness P] doubles, [max taumax bits] u64, [status P] int32
-  unsigned char* d_res = nullptr;
-  unsigned char* h_res = nullptr;  // pinned staging copy (small and medium result sets only)
-  unsigned char* h_stage[2] = {nullptr, nullptr};  // large result sets: two pinned chunks, copy-out pipelined
+  DeviceArray<unsigned char> d_res;
+  PinnedArray<unsigned char> h_res;  // pinned staging copy (small and medium result sets only)
+  // staged copies (ensure_stage): two pinned chunks of stage_bytes, copy-out and uploads pipelined
+  PinnedArray<unsigned char> h_stage[2];
+  Event stage_ev[2];
   size_t stage_bytes = 0;
-  cudaEvent_t stage_ev[2]{};
   bool stage_busy[2] = {false, false};  // an upload out of the chunk is in flight (staged_copy_in)
-  size_t res_bytes = 0;
   double *d_tau = nullptr, *d_p = nullptr, *d_tm = nullptr, *d_comp = nullptr;
   unsigned long long* d_maxbits = nullptr;
   int32_t* d_status = nullptr;
-  int64_t* d_counts = nullptr;
-  unsigned long long* d_scalars = nullptr;  // [0] unit counter, [1] max taumax bits
-  uint32_t* d_naive = nullptr;
+  DeviceArray<int64_t> d_counts;
+  DeviceArray<unsigned long long> d_scalars;  // [0] unit counter, [1] max taumax bits
+  DeviceArray<unsigned char> d_naive;
   int64_t naive_threads = 0;
-  // matrix output (icikt_plan_download_matrices), allocated on first use
-  double* d_mat = nullptr;          // 5 x [C][C]: cor, raw, pvalue, taumax, completeness (multi-GPU: 5 blocks of columns)
-  size_t mat_elems = 0;             // doubles allocated at d_mat
-  unsigned char* h_mat = nullptr;   // pinned copy of all five (small C only)
-  unsigned long long* d_hist = nullptr;  // [16] pairs per status class
-  int32_t* d_ngood = nullptr;       // [C] caller-supplied n_good
+  // matrix output (ensure_matrix_buffers), allocated on first use
+  DeviceArray<double> d_mat;          // 5 x [C][C]: cor, raw, pvalue, taumax, completeness (multi-GPU: 5 blocks of columns)
+  PinnedArray<unsigned char> h_mat;   // pinned copy of all five (small C only)
+  DeviceArray<unsigned long long> d_hist;  // [16] pairs per status class
+  DeviceArray<int32_t> d_ngood;       // [C] caller-supplied n_good
   bool pairs_done = false;
 
   // Pipelined one-shot call (staged plans only, see build_stage_table / run_staged): the pair order is cut
@@ -247,122 +267,48 @@ struct icikt_plan {
   bool staged = false;
   bool staged_run = false;               // the last run went through run_staged (selects the timing sums)
   std::vector<StageLaunch> stages;
-  cudaStream_t copy_stream = nullptr;    // uploads and downloads of a staged run
-  std::vector<cudaEvent_t> sync_ev;      // per launch: [2l] its columns have landed, [2l+1] its results are ready
-  std::vector<cudaEvent_t> time_ev;      // per launch: K1 start/end, K2 start, K2 end, K3 end
+  std::vector<Event> sync_ev;            // per launch: [2l] its columns have landed, [2l+1] its results are ready
+  std::vector<Event> time_ev;            // per launch: K1 start/end, K2 start, K2 end, K3 end
 
   // Filtered all-pairs call (icikt_all_pairs_edges, see run_edges): the plan's pair buffers hold one window of
   // the pair order; units, selected rows and the per-window readback are double-buffered.
-  PairUnit* d_wunits[2] = {nullptr, nullptr};
-  PairUnit* h_wunits[2] = {nullptr, nullptr};  // pinned
-  size_t wunit_cap = 0;
-  uint32_t* d_emask = nullptr;
-  uint32_t* d_etile = nullptr;
-  EdgeRow* d_erows[2] = {nullptr, nullptr};
-  unsigned long long* d_etotal = nullptr;  // [2]
-  unsigned long long* h_estat = nullptr;   // pinned [2][2]: rows kept, max taumax bits so far
-  cudaEvent_t eev[2][6]{};                 // per buffer: units up start/end, K2 start, K2 end, K3 end, selection end
+  DeviceArray<PairUnit> d_wunits[2];
+  PinnedArray<PairUnit> h_wunits[2];
+  DeviceArray<uint32_t> d_emask;
+  DeviceArray<uint32_t> d_etile;
+  DeviceArray<EdgeRow> d_erows[2];
+  DeviceArray<unsigned long long> d_etotal;  // [2]
+  PinnedArray<unsigned long long> h_estat;   // [2][2]: rows kept, max taumax bits so far
+  Event eev[2][6];                           // per buffer: units up start/end, K2 start, K2 end, K3 end, selection end
   // Top-k all-pairs call (icikt_all_pairs_topk), on the same window walk: per-column candidate counts, the
   // candidates of one window, and the lists of the L columns that keep one (all C, or one side of a cross call)
-  uint32_t* d_tcount = nullptr;
-  uint2* d_tcand = nullptr;    // [2 W]
-  TopkCol* d_tcol = nullptr;   // [L]
-  int32_t* d_tidx = nullptr;   // [L k]
-  double* d_tlist = nullptr;   // 4 x [L k]: raw, pvalue, taumax, completeness
-  int64_t topk_cols = 0;       // L d_tcount / d_tcol hold
-  int64_t topk_entries = 0;    // L k d_tidx / d_tlist hold
+  DeviceArray<uint32_t> d_tcount;  // [L]
+  DeviceArray<uint2> d_tcand;      // [2 W]
+  DeviceArray<TopkCol> d_tcol;     // [L]
+  DeviceArray<int32_t> d_tidx;     // [L k]
+  DeviceArray<double> d_tlist;     // 4 x [L k]: raw, pvalue, taumax, completeness
   // Cross per-pair call (icikt_cross_pairs): a window's results, moved off the pair buffers so that they can be
   // copied out while the next window runs; [tau W][pvalue W][taumax W][completeness W] doubles, [status W] int32
-  unsigned char* d_cres[2] = {nullptr, nullptr};
+  DeviceArray<unsigned char> d_cres[2];
   // Top-k over several devices (icikt_all_pairs_topk_multi): this device's block of columns of the merged lists
-  int32_t* d_mn = nullptr;     // [C] entries kept per column of the block
-  int32_t* d_midx = nullptr;   // [merge_cap]
-  double* d_mlist = nullptr;   // 4 x [merge_cap]: raw, pvalue, taumax, completeness
-  size_t merge_cap = 0;
+  DeviceArray<int32_t> d_mn;     // [C] entries kept per column of the block
+  DeviceArray<int32_t> d_midx;   // [entries]
+  DeviceArray<double> d_mlist;   // 4 x [entries]: raw, pvalue, taumax, completeness
 
-  cudaEvent_t ev[9]{};
+  Event ev[9];
   icikt_timings tm{};
+
+  // A failed call may leave copies in flight: none may still read a caller's array once the plan is gone.  The
+  // handles then release themselves on the plan's device.
+  ~icikt_plan() {
+    cudaSetDevice(device);
+    if (copy_stream) cudaStreamSynchronize(copy_stream);
+    if (stream) cudaStreamSynchronize(stream);
+    cudaGetLastError();
+  }
 };
 
 namespace {
-
-void free_plan(icikt_plan* p) {
-  if (!p) return;
-  cudaSetDevice(p->device);
-  // a failed call may leave copies in flight: none may still read a caller's array once the call returns
-  if (p->copy_stream) cudaStreamSynchronize(p->copy_stream);
-  if (p->stream) cudaStreamSynchronize(p->stream);
-  cudaGetLastError();
-  cudaFree(p->d_data_own);
-  cudaFree(p->d_global_na);
-  cudaFree(p->d_colptr);
-  cudaFree(p->d_rowidx);
-  cudaFree(p->d_values);
-  cudaFree(p->tab.perm);
-  cudaFree(p->tab.rank);
-  cudaFree(p->tab.trow);
-  cudaFree(p->tab.trun);
-  cudaFree(p->tab.tend);
-  cudaFree(p->tab.tord);
-  cudaFree(p->tab.nabits);
-  cudaFree(p->tab.firstbits);
-  cudaFree(p->tab.gstart);
-  cudaFree(p->tab.lgrp);
-  cudaFree(p->tab.stats);
-  cudaFree(p->tab.max_tied);
-  cudaFree(p->wk.keys_in);
-  cudaFree(p->wk.keys_out);
-  cudaFree(p->wk.vals_in);
-  cudaFree(p->wk.gpos);
-  cudaFree(p->d_units);
-  cudaFree(p->d_pj);
-  cudaFree(p->d_raw);
-  cudaFree(p->d_pw);
-  cudaFree(p->d_res);
-  if (p->h_res) cudaFreeHost(p->h_res);
-  for (int i = 0; i < 2; ++i) {
-    if (p->h_stage[i]) cudaFreeHost(p->h_stage[i]);
-    if (p->stage_ev[i]) cudaEventDestroy(p->stage_ev[i]);
-  }
-  cudaFree(p->d_counts);
-  cudaFree(p->d_scalars);
-  cudaFree(p->d_naive);
-  cudaFree(p->d_scratch);
-  cudaFree(p->d_mat);
-  if (p->h_mat) cudaFreeHost(p->h_mat);
-  cudaFree(p->d_hist);
-  cudaFree(p->d_ngood);
-  for (int b = 0; b < 2; ++b) {
-    cudaFree(p->d_wunits[b]);
-    if (p->h_wunits[b]) cudaFreeHost(p->h_wunits[b]);
-    cudaFree(p->d_erows[b]);
-    for (auto& e : p->eev[b])
-      if (e) cudaEventDestroy(e);
-  }
-  cudaFree(p->d_emask);
-  cudaFree(p->d_etile);
-  cudaFree(p->d_etotal);
-  if (p->h_estat) cudaFreeHost(p->h_estat);
-  cudaFree(p->d_tcount);
-  cudaFree(p->d_cres[0]);
-  cudaFree(p->d_cres[1]);
-  cudaFree(p->d_tcand);
-  cudaFree(p->d_tcol);
-  cudaFree(p->d_tidx);
-  cudaFree(p->d_tlist);
-  cudaFree(p->d_mn);
-  cudaFree(p->d_midx);
-  cudaFree(p->d_mlist);
-  for (auto& e : p->ev)
-    if (e) cudaEventDestroy(e);
-  for (auto& e : p->sync_ev)
-    if (e) cudaEventDestroy(e);
-  for (auto& e : p->time_ev)
-    if (e) cudaEventDestroy(e);
-  if (p->copy_stream) cudaStreamDestroy(p->copy_stream);
-  if (p->stream) cudaStreamDestroy(p->stream);
-  delete p;
-}
 
 // The units of pairs [lo, hi) of the all-pairs order of C columns (combn order, then the diagonal if
 // include_diag), appended to U with slots counted from lo.  `first_row`: a row at or before the row of pair lo
@@ -495,12 +441,12 @@ int staged_copy_out(icikt_plan* p, void* dst, const void* d_src, size_t bytes, c
     const int cur = k & 1;
     if (len[cur]) {  // the chunk issued two steps ago has landed in h_stage[cur]
       CK(cudaEventSynchronize(p->stage_ev[cur]));
-      host_copy(out + off[cur], p->h_stage[cur], len[cur]);
+      host_copy(out + off[cur], p->h_stage[cur].get(), len[cur]);
       len[cur] = 0;
     }
     if (o < bytes) {
       const size_t l = std::min(p->stage_bytes, bytes - o);
-      CK(cudaMemcpyAsync(p->h_stage[cur], src + o, l, cudaMemcpyDeviceToHost, stream));
+      CK(cudaMemcpyAsync(p->h_stage[cur].get(), src + o, l, cudaMemcpyDeviceToHost, stream));
       CK(cudaEventRecord(p->stage_ev[cur], stream));
       off[cur] = o;
       len[cur] = l;
@@ -510,12 +456,12 @@ int staged_copy_out(icikt_plan* p, void* dst, const void* d_src, size_t bytes, c
   return ICIKT_OK;
 }
 
+// the two pinned chunks of the staged copies and their events (kept with the plan)
 int ensure_stage(icikt_plan* p) {
-  if (p->h_stage[0]) return ICIKT_OK;
-  p->stage_bytes = stage_chunk();
+  if (!p->stage_bytes) p->stage_bytes = stage_chunk();
   for (int i = 0; i < 2; ++i) {
-    CK(cudaMallocHost(reinterpret_cast<void**>(&p->h_stage[i]), p->stage_bytes));
-    CK(cudaEventCreateWithFlags(&p->stage_ev[i], cudaEventDisableTiming));
+    ECK(p->h_stage[i].reserve(p->stage_bytes));
+    if (!p->stage_ev[i]) ECK(p->stage_ev[i].create(cudaEventDisableTiming));
   }
   return ICIKT_OK;
 }
@@ -537,8 +483,8 @@ int staged_copy_in(icikt_plan* p, void* d_dst, const void* src, size_t bytes, cu
       p->stage_busy[cur] = false;
     }
     const size_t l = std::min(p->stage_bytes, bytes - o);
-    host_copy(p->h_stage[cur], in + o, l);
-    CK(cudaMemcpyAsync(dst + o, p->h_stage[cur], l, cudaMemcpyHostToDevice, stream));
+    host_copy(p->h_stage[cur].get(), in + o, l);
+    CK(cudaMemcpyAsync(dst + o, p->h_stage[cur].get(), l, cudaMemcpyHostToDevice, stream));
     CK(cudaEventRecord(p->stage_ev[cur], stream));
     p->stage_busy[cur] = true;
     o += l;
@@ -661,25 +607,19 @@ int copy_array_in(icikt_plan* p, void* d_dst, const void* src, size_t bytes, cud
 // value the expansion of the first chunk may be reading.)
 int copy_csc_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, int64_t dst, cudaStream_t stream) {
   const int64_t nnz = s.colptr[s.C];
-  if (!p->d_colptr) CK(dmalloc(&p->d_colptr, (size_t)p->C + 1));
-  if (nnz > p->csc_cap) {  // nothing of an earlier call is in flight: every call ends with its streams idle
-    cudaFree(p->d_rowidx);
-    cudaFree(p->d_values);
-    p->d_rowidx = nullptr;
-    p->d_values = nullptr;
-    p->csc_cap = 0;
-    CK(dmalloc(&p->d_rowidx, (size_t)nnz));
-    CK(dmalloc(&p->d_values, (size_t)nnz));
-    p->csc_cap = nnz;
+  CK(p->d_colptr.reserve((size_t)p->C + 1));
+  if (nnz > 0) {  // nothing of an earlier call is in flight: every call ends with its streams idle
+    CK(p->d_rowidx.reserve((size_t)nnz));
+    CK(p->d_values.reserve((size_t)nnz));
   }
   p->expand_lo = p->expand_hi = 0;
   if (c_hi <= c_lo) return ICIKT_OK;
   const int64_t k_lo = s.colptr[c_lo], k_hi = s.colptr[c_hi];
-  CK(cudaMemcpyAsync(p->d_colptr + c_lo, s.colptr + c_lo, sizeof(int64_t) * (size_t)(c_hi - c_lo + 1),
+  CK(cudaMemcpyAsync(p->d_colptr.get() + c_lo, s.colptr + c_lo, sizeof(int64_t) * (size_t)(c_hi - c_lo + 1),
                      cudaMemcpyHostToDevice, stream));
-  int rc = copy_array_in(p, p->d_rowidx + k_lo, s.rowidx + k_lo, sizeof(int32_t) * (size_t)(k_hi - k_lo), stream);
+  int rc = copy_array_in(p, p->d_rowidx.get() + k_lo, s.rowidx + k_lo, sizeof(int32_t) * (size_t)(k_hi - k_lo), stream);
   if (rc == ICIKT_OK)
-    rc = copy_array_in(p, p->d_values + k_lo, s.values + k_lo, sizeof(double) * (size_t)(k_hi - k_lo), stream);
+    rc = copy_array_in(p, p->d_values.get() + k_lo, s.values + k_lo, sizeof(double) * (size_t)(k_hi - k_lo), stream);
   if (rc != ICIKT_OK) return rc;
   p->expand_lo = c_lo;
   p->expand_hi = c_hi;
@@ -691,13 +631,13 @@ int copy_csc_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi
 // [dst + c_lo, dst + c_hi) (CSC: of their stored entries), on `stream`
 int copy_columns_in(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c_hi, cudaStream_t stream,
                     int64_t dst = 0) {
-  if (!p->d_data_own) CK(dmalloc(&p->d_data_own, (size_t)p->n * p->C));
+  CK(p->d_data_own.reserve((size_t)p->n * p->C));
   if (s.csc()) return copy_csc_in(p, s, c_lo, c_hi, dst, stream);
   p->expand_lo = p->expand_hi = 0;
   const double* data = s.data;
   const int64_t ld = s.ld;
   if (c_hi <= c_lo) return ICIKT_OK;
-  double* out = p->d_data_own + (size_t)(dst + c_lo) * p->n;
+  double* out = p->d_data_own.get() + (size_t)(dst + c_lo) * p->n;
   const size_t bytes = sizeof(double) * (size_t)p->n * (size_t)(c_hi - c_lo);
   if (ld == p->n && bytes >= (8u << 20) && !std::getenv("ICIKT_NO_STAGED_UPLOAD") && !host_is_pinned(data + (size_t)c_lo * ld))
     return staged_copy_in(p, out, data + (size_t)c_lo * ld, bytes, stream);
@@ -712,7 +652,7 @@ int upload_columns(icikt_plan* p, const ColumnSource& s, int64_t c_lo, int64_t c
   const int rc = copy_columns_in(p, s, c_lo, c_hi, p->stream);
   if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[1], p->stream));
-  p->d_data = p->d_data_own;
+  p->d_data = p->d_data_own.get();
   p->ld = p->n;
   p->columns_done = false;
   p->pairs_done = false;
@@ -741,6 +681,18 @@ class HostBarrier {
   std::condition_variable cv_;
   int n_, count_ = 0, gen_ = 0;
 };
+
+// the matrix fill's buffers (kept with the plan): `elems` doubles of matrices (`what` names them in the error), the
+// status histogram and n_good
+int ensure_matrix_buffers(icikt_plan* p, size_t elems, const char* what) {
+  if (p->d_mat.reserve(elems) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ICIKT_ERR_ALLOC, std::string("device allocation of ") + what + " failed");
+  }
+  CK(p->d_hist.reserve(16));
+  CK(p->d_ngood.reserve((size_t)p->C));
+  return ICIKT_OK;
+}
 
 // elapsed time between two completed events; 0 if one of them was never recorded
 float ev_ms(cudaEvent_t a, cudaEvent_t b) {
@@ -791,7 +743,7 @@ static int plan_create_impl(icikt_plan** out, int64_t n, int64_t C, const int32_
   int rc = select_device(o.device);
   if (rc != ICIKT_OK) return rc;
 
-  icikt_plan* p = new (std::nothrow) icikt_plan();
+  std::unique_ptr<icikt_plan> p(new (std::nothrow) icikt_plan());
   if (!p) return fail(ICIKT_ERR_ALLOC, "out of host memory");
   p->device = o.device;
   p->opts = o;
@@ -799,14 +751,12 @@ static int plan_create_impl(icikt_plan** out, int64_t n, int64_t C, const int32_
   p->n = n;
   p->C = C;
   cudaDeviceProp prop;
-  if (cudaGetDeviceProperties(&prop, o.device) != cudaSuccess) { free_plan(p); return fail(ICIKT_ERR_CUDA, "cudaGetDeviceProperties failed"); }
+  if (cudaGetDeviceProperties(&prop, o.device) != cudaSuccess) return fail(ICIKT_ERR_CUDA, "cudaGetDeviceProperties failed");
   p->n_sm = prop.multiProcessorCount;
-  if (prop.major < 10) {
-    free_plan(p);
+  if (prop.major < 10)
     return fail(ICIKT_ERR_NO_DEVICE, "device is not sm_100-class; this library is built for sm_100a only");
-  }
   if (staged) {
-    if (pi || o.pair_lo != 0 || o.pair_hi != 0) { free_plan(p); return fail(ICIKT_ERR_BAD_ARG, "staged plans cover all pairs"); }
+    if (pi || o.pair_lo != 0 || o.pair_hi != 0) return fail(ICIKT_ERR_BAD_ARG, "staged plans cover all pairs");
     p->staged = true;
     p->P = tri_pairs(C) + (o.include_diag ? C : 0);
     // row blocks of the last chunk: the copy-out of the final block is all that stays exposed
@@ -814,101 +764,87 @@ static int plan_create_impl(icikt_plan** out, int64_t n, int64_t C, const int32_
     if (const char* e = std::getenv("ICIKT_PIPELINE_BLOCKS")) blocks = std::max(1, std::min(64, std::atoi(e)));
     build_stage_table(C, o.include_diag != 0, (int64_t)p->n_sm * 2, blocks, p->units, p->stages);
   } else {
-    rc = build_units(p, pi, pj, P);
-    if (rc != ICIKT_OK) { free_plan(p); return rc; }
+    rc = build_units(p.get(), pi, pj, P);
+    if (rc != ICIKT_OK) return rc;
   }
   for (const PairUnit& u : p->units) p->max_unit_pairs = std::max(p->max_unit_pairs, (int)u.count);
 
-#define PCK(call)                                                \
-  do {                                                           \
-    cudaError_t e_ = (call);                                     \
-    if (e_ != cudaSuccess) {                                     \
-      const int c_ = (e_ == cudaErrorMemoryAllocation) ? fail(ICIKT_ERR_ALLOC, "device allocation failed: " #call) \
-                                                       : cuda_fail(e_, #call);                     \
-      free_plan(p);                                              \
-      return c_;                                                 \
-    }                                                            \
-  } while (0)
-
-  PCK(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
-  for (auto& e : p->ev) PCK(cudaEventCreate(&e));
+  ECK(p->stream.create());
+  for (Event& e : p->ev) ECK(e.create());
   if (staged) {
-    PCK(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
-    p->sync_ev.assign(2 * p->stages.size(), nullptr);
-    p->time_ev.assign(5 * p->stages.size(), nullptr);
-    for (auto& e : p->sync_ev) PCK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    for (auto& e : p->time_ev) PCK(cudaEventCreate(&e));
+    ECK(p->copy_stream.create());
+    p->sync_ev.resize(2 * p->stages.size());
+    p->time_ev.resize(5 * p->stages.size());
+    for (Event& e : p->sync_ev) ECK(e.create(cudaEventDisableTiming));
+    for (Event& e : p->time_ev) ECK(e.create());
   }
   ColumnTables& t = p->tab;
+  auto& m = p->col_mem;
   t.n = n;
   t.C = C;
   t.nstride = (n + 63) & ~63LL;
   const int64_t nwords = ((n + 31) & ~31LL) / 32;
   t.wstride = (nwords + 3) & ~3LL;
   const size_t ne = (size_t)t.nstride * C, nw = (size_t)t.wstride * C;
-  PCK(dmalloc(&t.perm, ne));
-  PCK(dmalloc(&t.rank, ne));
-  PCK(dmalloc(&t.trow, ne));
-  PCK(dmalloc(&t.trun, ne));
-  PCK(dmalloc(&t.tend, ne));
-  PCK(dmalloc(&t.tord, ne));
-  PCK(dmalloc(&t.nabits, nw));
-  PCK(dmalloc(&t.firstbits, nw));
+  ECK(reserve_view(m.perm, t.perm, ne));
+  ECK(reserve_view(m.rank, t.rank, ne));
+  ECK(reserve_view(m.trow, t.trow, ne));
+  ECK(reserve_view(m.trun, t.trun, ne));
+  ECK(reserve_view(m.tend, t.tend, ne));
+  ECK(reserve_view(m.tord, t.tord, ne));
+  ECK(reserve_view(m.nabits, t.nabits, nw));
+  ECK(reserve_view(m.firstbits, t.firstbits, nw));
   t.gstride = t.nstride + 64;
-  PCK(dmalloc(&t.gstart, (size_t)t.gstride * C));
-  PCK(dmalloc(&t.lgrp, (size_t)kLargeStride * C));
-  PCK(dmalloc(&t.stats, (size_t)C));
-  PCK(dmalloc(&t.max_tied, 4));
+  ECK(reserve_view(m.gstart, t.gstart, (size_t)t.gstride * C));
+  ECK(reserve_view(m.lgrp, t.lgrp, (size_t)kLargeStride * C));
+  ECK(reserve_view(m.stats, t.stats, (size_t)C));
+  ECK(reserve_view(m.max_tied, t.max_tied, 4));
   // padding words of the bit arrays (beyond n32/32) are never written by the kernels
-  PCK(cudaMemsetAsync(t.nabits, 0, sizeof(uint32_t) * nw, p->stream));
-  PCK(cudaMemsetAsync(t.firstbits, 0, sizeof(uint32_t) * nw, p->stream));
-  PCK(cudaMemsetAsync(t.max_tied, 0, 4 * sizeof(int32_t), p->stream));
+  ECK(cudaMemsetAsync(t.nabits, 0, sizeof(uint32_t) * nw, p->stream));
+  ECK(cudaMemsetAsync(t.firstbits, 0, sizeof(uint32_t) * nw, p->stream));
+  ECK(cudaMemsetAsync(t.max_tied, 0, 4 * sizeof(int32_t), p->stream));
   p->shape = tiled_shape(n, 0, t.wstride, p->n_sm);
   if (!columns_fused(n)) {  // scratch of the multi-kernel column path (long columns)
-    PCK(dmalloc(&p->wk.keys_in, ne));
-    PCK(dmalloc(&p->wk.keys_out, ne));
-    PCK(dmalloc(&p->wk.vals_in, ne));
-    PCK(dmalloc(&p->wk.gpos, (size_t)(t.nstride + 64) * C));
+    ECK(reserve_view(m.keys_in, p->wk.keys_in, ne));
+    ECK(reserve_view(m.keys_out, p->wk.keys_out, ne));
+    ECK(reserve_view(m.vals_in, p->wk.vals_in, ne));
+    ECK(reserve_view(m.gpos, p->wk.gpos, (size_t)(t.nstride + 64) * C));
   }
-  PCK(dmalloc(&p->d_global_na, 64));
+  ECK(p->d_global_na.reserve(64));
 
   const size_t np = (size_t)std::max<int64_t>(p->P, 1);
-  PCK(dmalloc(&p->d_units, p->units.size()));
-  PCK(cudaMemcpyAsync(p->d_units, p->units.data(), sizeof(PairUnit) * p->units.size(),
+  ECK(p->d_units.reserve(p->units.size()));
+  ECK(cudaMemcpyAsync(p->d_units.get(), p->units.data(), sizeof(PairUnit) * p->units.size(),
                       cudaMemcpyHostToDevice, p->stream));
   if (pi) {
-    PCK(dmalloc(&p->d_pj, np));
-    PCK(cudaMemcpyAsync(p->d_pj, pj, sizeof(int32_t) * np, cudaMemcpyHostToDevice, p->stream));
+    ECK(p->d_pj.reserve(np));
+    ECK(cudaMemcpyAsync(p->d_pj.get(), pj, sizeof(int32_t) * np, cudaMemcpyHostToDevice, p->stream));
   }
-  PCK(dmalloc(&p->d_raw, np));
-  if (o.perspective == ICIKT_PERSPECTIVE_COMPLETE) PCK(dmalloc(&p->d_pw, np));
-  p->res_bytes = np * (4 * sizeof(double) + sizeof(int32_t)) + sizeof(unsigned long long);
-  PCK(cudaMalloc(reinterpret_cast<void**>(&p->d_res), p->res_bytes));
-  p->d_tau = reinterpret_cast<double*>(p->d_res);
+  ECK(p->d_raw.reserve(np));
+  if (o.perspective == ICIKT_PERSPECTIVE_COMPLETE) ECK(p->d_pw.reserve(np));
+  const size_t res_bytes = np * (4 * sizeof(double) + sizeof(int32_t)) + sizeof(unsigned long long);
+  ECK(p->d_res.reserve(res_bytes));
+  p->d_tau = reinterpret_cast<double*>(p->d_res.get());
   p->d_p = p->d_tau + np;
   p->d_tm = p->d_p + np;
   p->d_comp = p->d_tm + np;
   p->d_maxbits = reinterpret_cast<unsigned long long*>(p->d_comp + np);
   p->d_status = reinterpret_cast<int32_t*>(p->d_maxbits + 1);
-  if (p->res_bytes <= stage_all()) {
-    PCK(cudaMallocHost(reinterpret_cast<void**>(&p->h_res), p->res_bytes));
+  if (res_bytes <= stage_all()) {
+    ECK(p->h_res.reserve(res_bytes));
   } else {
-    p->stage_bytes = stage_chunk();
-    for (int i = 0; i < 2; ++i) {
-      PCK(cudaMallocHost(reinterpret_cast<void**>(&p->h_stage[i]), p->stage_bytes));
-      PCK(cudaEventCreateWithFlags(&p->stage_ev[i], cudaEventDisableTiming));
-    }
+    rc = ensure_stage(p.get());
+    if (rc != ICIKT_OK) return rc;
   }
-  if (p->want_counts) PCK(dmalloc(&p->d_counts, np * ICIKT_NCOUNTS));
-  PCK(dmalloc(&p->d_scalars, 2));  // [0] unit counter
+  if (p->want_counts) ECK(p->d_counts.reserve(np * ICIKT_NCOUNTS));
+  ECK(p->d_scalars.reserve(2));  // [0] unit counter
   if (o.kernel == ICIKT_KERNEL_NAIVE) {
     p->naive_threads = std::min<int64_t>((int64_t)p->units.size(), (int64_t)p->n_sm * 256);
     p->naive_threads = std::max<int64_t>(p->naive_threads, 1);
-    PCK(cudaMalloc(reinterpret_cast<void**>(&p->d_naive), naive_scratch_bytes(n, p->naive_threads)));
+    ECK(p->d_naive.reserve(naive_scratch_bytes(n, p->naive_threads)));
   }
-  PCK(cudaStreamSynchronize(p->stream));  // pj / units are read from caller memory
-#undef PCK
-  *out = p;
+  ECK(cudaStreamSynchronize(p->stream));  // pj / units are read from caller memory
+  *out = p.release();
   return ICIKT_OK;
 }
 
@@ -941,8 +877,8 @@ int icikt_plan_set_device_matrix(icikt_plan* p, const double* d_data, int64_t ld
 // launches or < 0 (the error is set)
 static int expand_columns(icikt_plan* p) {
   if (p->expand_hi <= p->expand_lo) return 0;
-  const int l = launch_csc_expand(p->d_colptr, p->d_rowidx, p->d_values, p->n, p->expand_lo, p->expand_hi,
-                                  p->d_data_own + (size_t)p->expand_dst * p->n, p->stream);
+  const int l = launch_csc_expand(p->d_colptr.get(), p->d_rowidx.get(), p->d_values.get(), p->n, p->expand_lo, p->expand_hi,
+                                  p->d_data_own.get() + (size_t)p->expand_dst * p->n, p->stream);
   if (l < 0) return launch_fail("CSC expansion kernel"), -1;
   p->expand_lo = p->expand_hi = p->expand_dst = 0;
   return l;
@@ -969,7 +905,7 @@ static int plan_columns_impl(icikt_plan* p, const double* global_na, int32_t n_g
     if (nlit == 64) return fail(ICIKT_ERR_BAD_ARG, "more than 64 global_na literals");
     lit[nlit++] = v;
   }
-  if (nlit) CK(cudaMemcpyAsync(p->d_global_na, lit, sizeof(double) * nlit, cudaMemcpyHostToDevice, p->stream));
+  if (nlit) CK(cudaMemcpyAsync(p->d_global_na.get(), lit, sizeof(double) * nlit, cudaMemcpyHostToDevice, p->stream));
   if (reset) CK(cudaMemsetAsync(p->tab.max_tied, 0, 4 * sizeof(int32_t), p->stream));
   CK(cudaEventRecord(e0 ? e0 : p->ev[2], p->stream));
   // columns uploaded as CSC become dense first (their copies precede this point on the stream)
@@ -986,23 +922,21 @@ static int plan_columns_impl(icikt_plan* p, const double* global_na, int32_t n_g
   const int slot_ctas = std::max(std::max(worst.max_ctas, p->shape.max_ctas), std::max(p->shape_mid.max_ctas, p->n_sm * 2));
   const bool any_gmem = worst.gmem || worst.const_gmem || p->shape.gmem || p->shape_mid.gmem;
   const size_t need = (size_t)slot_ctas * (size_t)slot_bytes;
-  if (any_gmem && need > p->scratch_bytes) {
+  if (any_gmem && need > p->d_scratch.size()) {
     // the shape depends on the perspective class and on tuning knobs in the environment, so a cached
     // plan may need a larger scratch than the one it was given first
     CK(cudaStreamSynchronize(p->stream));
-    if (p->d_scratch) { cudaFree(p->d_scratch); p->d_scratch = nullptr; p->scratch_bytes = 0; }
-    if (cudaMalloc(reinterpret_cast<void**>(&p->d_scratch), need) != cudaSuccess) {
+    if (p->d_scratch.reserve(need) != cudaSuccess) {
       cudaGetLastError();
       return fail(ICIKT_ERR_ALLOC, "device allocation of the pair kernel's global scratch failed");
     }
-    p->scratch_bytes = need;
   }
   for (TiledShape* sh : {&p->shape, &p->shape_mid, &p->shape_heavy}) {
     sh->scratch_stride = p->d_scratch ? slot_bytes : 0;
-    sh->scratch_ctas = p->d_scratch ? (int)std::min<size_t>((size_t)slot_ctas, p->scratch_bytes / (size_t)slot_bytes) : 0;
+    sh->scratch_ctas = p->d_scratch ? (int)std::min<size_t>((size_t)slot_ctas, p->d_scratch.size() / (size_t)slot_bytes) : 0;
   }
-  const int lc = launch_columns(p->d_data, p->ld, p->d_global_na, nlit, na_inf, p->tab, p->wk, p->shape,
-                                p->d_scratch, p->stream, col_lo, col_hi);
+  const int lc = launch_columns(p->d_data, p->ld, p->d_global_na.get(), nlit, na_inf, p->tab, p->wk, p->shape,
+                                p->d_scratch.get(), p->stream, col_lo, col_hi);
   if (lc < 0) return launch_fail("column kernels");
   const int l = lc + expand_launches;
   CK(cudaEventRecord(e1 ? e1 : p->ev[3], p->stream));
@@ -1076,17 +1010,17 @@ int icikt_plan_tables(icikt_plan* p, icikt_table* out, int32_t cap) {
 // bracket K2 and K3 on the plan's stream
 static int launch_pair_group(icikt_plan* p, const PairUnit* units, int64_t unit_lo, int64_t unit_hi, int max_unit_pairs, cudaEvent_t e_start,
                              cudaEvent_t e_mid, cudaEvent_t e_end, int* launches_out) {
-  CK(cudaMemsetAsync(p->d_scalars, 0, 2 * sizeof(unsigned long long), p->stream));
+  CK(cudaMemsetAsync(p->d_scalars.get(), 0, 2 * sizeof(unsigned long long), p->stream));
   CK(cudaEventRecord(e_start, p->stream));
   PairLaunch pl;
   pl.tab = &p->tab;
   pl.units = units + unit_lo;
   pl.n_units = unit_hi - unit_lo;
-  pl.pj_list = p->d_pj;
-  pl.raw = p->d_raw;
-  pl.pw = (p->opts.perspective == ICIKT_PERSPECTIVE_COMPLETE) ? p->d_pw : nullptr;
-  pl.unit_counter = p->d_scalars;
-  pl.scratch = p->d_scratch;
+  pl.pj_list = p->d_pj.get();
+  pl.raw = p->d_raw.get();
+  pl.pw = (p->opts.perspective == ICIKT_PERSPECTIVE_COMPLETE) ? p->d_pw.get() : nullptr;
+  pl.unit_counter = p->d_scalars.get();
+  pl.scratch = p->d_scratch.get();
   int launches = 0;
   if (pl.n_units <= 0) {
     CK(cudaEventRecord(e_mid, p->stream));
@@ -1095,7 +1029,7 @@ static int launch_pair_group(icikt_plan* p, const PairUnit* units, int64_t unit_
     if (pl.pw && p->opts.kernel == ICIKT_KERNEL_NAIVE)
       return fail(ICIKT_ERR_BAD_ARG, "the complete-observations mode needs the tiled kernel");
     if (p->opts.kernel == ICIKT_KERNEL_NAIVE)
-      l = launch_pairs_naive(pl, p->P, p->d_naive, p->naive_threads, p->stream);
+      l = launch_pairs_naive(pl, p->P, reinterpret_cast<uint32_t*>(p->d_naive.get()), p->naive_threads, p->stream);
     else {
       l = launch_pairs_tiled(pl, p->shape, p->n_sm, 0, p->stream);
       if (l > 0) {
@@ -1118,8 +1052,8 @@ static int launch_pair_group(icikt_plan* p, const PairUnit* units, int64_t unit_
     el.units = pl.units;
     el.n_units = pl.n_units;
     el.max_unit_pairs = max_unit_pairs;
-    el.pj_list = p->d_pj;
-    el.raw = p->d_raw;
+    el.pj_list = p->d_pj.get();
+    el.raw = p->d_raw.get();
     el.pw = pl.pw;
     el.perspective = p->opts.perspective;
     el.alternative = p->opts.alternative;
@@ -1129,7 +1063,7 @@ static int launch_pair_group(icikt_plan* p, const PairUnit* units, int64_t unit_
     el.taumax = p->d_tm;
     el.completeness = p->d_comp;
     el.status = p->d_status;
-    el.counts = p->d_counts;
+    el.counts = p->d_counts.get();
     el.max_taumax_bits = p->d_maxbits;
     l = launch_epilogue(el, p->stream);
     if (l < 0) return launch_fail("epilogue kernel");
@@ -1145,7 +1079,7 @@ int icikt_plan_pairs(icikt_plan* p) {
   CK(cudaSetDevice(p->device));
   CK(cudaMemsetAsync(p->d_maxbits, 0, sizeof(unsigned long long), p->stream));
   int launches = 0;
-  const int rc = launch_pair_group(p, p->d_units, 0, (int64_t)p->units.size(), p->max_unit_pairs, p->ev[4], p->ev[8], p->ev[5], &launches);
+  const int rc = launch_pair_group(p, p->d_units.get(), 0, (int64_t)p->units.size(), p->max_unit_pairs, p->ev[4], p->ev[8], p->ev[5], &launches);
   if (rc != ICIKT_OK) return rc;
   p->tm.n_launches = (p->tm.n_launches & 0xffff) | (launches << 16);
   p->pairs_done = true;
@@ -1170,18 +1104,18 @@ int icikt_plan_download(icikt_plan* p, double* raw, double* pvalue, double* taum
   unsigned long long bits = 0;
   if (p->h_res) {
     // one device-to-host copy into pinned memory, then plain host copies into the caller's arrays
-    CK(cudaMemcpyAsync(p->h_res, p->d_res, p->res_bytes, cudaMemcpyDeviceToHost, p->stream));
-    if (counts && np) CK(cudaMemcpyAsync(counts, p->d_counts, sizeof(int64_t) * np * ICIKT_NCOUNTS, cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaMemcpyAsync(p->h_res.get(), p->d_res.get(), p->d_res.size(), cudaMemcpyDeviceToHost, p->stream));
+    if (counts && np) CK(cudaMemcpyAsync(counts, p->d_counts.get(), sizeof(int64_t) * np * ICIKT_NCOUNTS, cudaMemcpyDeviceToHost, p->stream));
     CK(cudaEventRecord(p->ev[7], p->stream));
     CK(cudaStreamSynchronize(p->stream));
     const size_t npad = std::max<size_t>(np, 1);
-    const double* h = reinterpret_cast<const double*>(p->h_res);
+    const double* h = reinterpret_cast<const double*>(p->h_res.get());
     if (np) {
       if (raw) host_copy(raw, h, sizeof(double) * np);
       if (pvalue) host_copy(pvalue, h + npad, sizeof(double) * np);
       if (taumax) host_copy(taumax, h + 2 * npad, sizeof(double) * np);
       if (completeness) host_copy(completeness, h + 3 * npad, sizeof(double) * np);
-      if (status) host_copy(status, p->h_res + 4 * npad * sizeof(double) + sizeof(unsigned long long), sizeof(int32_t) * np);
+      if (status) host_copy(status, p->h_res.get() + 4 * npad * sizeof(double) + sizeof(unsigned long long), sizeof(int32_t) * np);
     }
     std::memcpy(&bits, h + 4 * npad, sizeof(bits));
   } else {
@@ -1192,7 +1126,7 @@ int icikt_plan_download(icikt_plan* p, double* raw, double* pvalue, double* taum
       if (rc == ICIKT_OK && taumax) rc = staged_copy_out(p, taumax, p->d_tm, sizeof(double) * np, p->stream);
       if (rc == ICIKT_OK && completeness) rc = staged_copy_out(p, completeness, p->d_comp, sizeof(double) * np, p->stream);
       if (rc == ICIKT_OK && status) rc = staged_copy_out(p, status, p->d_status, sizeof(int32_t) * np, p->stream);
-      if (rc == ICIKT_OK && counts) rc = staged_copy_out(p, counts, p->d_counts, sizeof(int64_t) * np * ICIKT_NCOUNTS, p->stream);
+      if (rc == ICIKT_OK && counts) rc = staged_copy_out(p, counts, p->d_counts.get(), sizeof(int64_t) * np * ICIKT_NCOUNTS, p->stream);
       if (rc != ICIKT_OK) return rc;
     }
     CK(cudaMemcpyAsync(&bits, p->d_maxbits, sizeof(bits), cudaMemcpyDeviceToHost, p->stream));
@@ -1214,18 +1148,8 @@ int icikt_plan_download_matrices(icikt_plan* p, int32_t scale_max, int32_t diag_
   CK(cudaSetDevice(p->device));
   const size_t C = (size_t)p->C, cc = C * C;
   double* outs[5] = {cor, raw, pvalue, taumax, completeness};
-  if (p->mat_elems < 5 * cc) {
-    cudaFree(p->d_mat);
-    p->d_mat = nullptr;
-    p->mat_elems = 0;
-    if (dmalloc(&p->d_mat, 5 * cc) != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ICIKT_ERR_ALLOC, "device allocation of the result matrices failed");
-    }
-    p->mat_elems = 5 * cc;
-  }
-  if (!p->d_hist) CK(dmalloc(&p->d_hist, 16));
-  if (!p->d_ngood) CK(dmalloc(&p->d_ngood, C));
+  int rc = ensure_matrix_buffers(p, 5 * cc, "the result matrices");
+  if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[6], p->stream));
   // entries no pair writes stay 0 (R/kendalltau.R:389-396 start from matrix(0, ...)); with every pair
   // and the diagonal present nothing needs clearing
@@ -1233,15 +1157,15 @@ int icikt_plan_download_matrices(icikt_plan* p, int32_t scale_max, int32_t diag_
   const bool covered = !p->d_pj && p->P == ptot && (p->opts.include_diag || diag_good);
   MatrixFill mf{};
   for (int k = 0; k < 5; ++k) {
-    mf.m[k] = outs[k] ? p->d_mat + (size_t)k * cc : nullptr;
+    mf.m[k] = outs[k] ? p->d_mat.get() + (size_t)k * cc : nullptr;
     if (outs[k] && !covered) CK(cudaMemsetAsync(mf.m[k], 0, sizeof(double) * cc, p->stream));
   }
-  CK(cudaMemsetAsync(p->d_hist, 0, 16 * sizeof(unsigned long long), p->stream));
-  if (n_good) CK(cudaMemcpyAsync(p->d_ngood, n_good, sizeof(int32_t) * C, cudaMemcpyHostToDevice, p->stream));
-  mf.units = p->d_units;
+  CK(cudaMemsetAsync(p->d_hist.get(), 0, 16 * sizeof(unsigned long long), p->stream));
+  if (n_good) CK(cudaMemcpyAsync(p->d_ngood.get(), n_good, sizeof(int32_t) * C, cudaMemcpyHostToDevice, p->stream));
+  mf.units = p->d_units.get();
   mf.n_units = (int64_t)p->units.size();
   mf.max_unit_pairs = p->max_unit_pairs;
-  mf.pj_list = p->d_pj;
+  mf.pj_list = p->d_pj.get();
   mf.tau = p->d_tau;
   mf.pvalue = p->d_p;
   mf.taumax = p->d_tm;
@@ -1249,37 +1173,32 @@ int icikt_plan_download_matrices(icikt_plan* p, int32_t scale_max, int32_t diag_
   mf.status = p->d_status;
   mf.max_taumax_bits = p->d_maxbits;
   mf.stats = p->tab.stats;
-  mf.n_good = n_good ? p->d_ngood : nullptr;
+  mf.n_good = n_good ? p->d_ngood.get() : nullptr;
   mf.n = p->n;
   mf.C = p->C;
   mf.scale_max = scale_max != 0;
   mf.diag_good = diag_good != 0;
-  mf.hist = p->d_hist;
+  mf.hist = p->d_hist.get();
   if (p->P <= 0) mf.n_units = 0;
   if (launch_matrix_fill(mf, p->stream) < 0) return launch_fail("matrix fill kernel");
   const size_t all_bytes = 5 * cc * sizeof(double);
   if (all_bytes <= stage_all()) {
-    if (!p->h_mat) CK(cudaMallocHost(reinterpret_cast<void**>(&p->h_mat), all_bytes));
+    CK(p->h_mat.reserve(all_bytes));
     for (int k = 0; k < 5; ++k)
       if (outs[k])
-        CK(cudaMemcpyAsync(p->h_mat + (size_t)k * cc * sizeof(double), mf.m[k], sizeof(double) * cc,
+        CK(cudaMemcpyAsync(p->h_mat.get() + (size_t)k * cc * sizeof(double), mf.m[k], sizeof(double) * cc,
                            cudaMemcpyDeviceToHost, p->stream));
     CK(cudaStreamSynchronize(p->stream));
     for (int k = 0; k < 5; ++k)
-      if (outs[k]) host_copy(outs[k], p->h_mat + (size_t)k * cc * sizeof(double), sizeof(double) * cc);
+      if (outs[k]) host_copy(outs[k], p->h_mat.get() + (size_t)k * cc * sizeof(double), sizeof(double) * cc);
   } else {
-    {
-      const int rc = ensure_stage(p);
-      if (rc != ICIKT_OK) return rc;
-    }
-    for (int k = 0; k < 5; ++k)
-      if (outs[k]) {
-        const int rc = staged_copy_out(p, outs[k], mf.m[k], sizeof(double) * cc, p->stream);
-        if (rc != ICIKT_OK) return rc;
-      }
+    rc = ensure_stage(p);
+    for (int k = 0; k < 5 && rc == ICIKT_OK; ++k)
+      if (outs[k]) rc = staged_copy_out(p, outs[k], mf.m[k], sizeof(double) * cc, p->stream);
+    if (rc != ICIKT_OK) return rc;
   }
   unsigned long long hist[16], bits = 0;
-  CK(cudaMemcpyAsync(hist, p->d_hist, sizeof(hist), cudaMemcpyDeviceToHost, p->stream));
+  CK(cudaMemcpyAsync(hist, p->d_hist.get(), sizeof(hist), cudaMemcpyDeviceToHost, p->stream));
   CK(cudaMemcpyAsync(&bits, p->d_maxbits, sizeof(bits), cudaMemcpyDeviceToHost, p->stream));
   CK(cudaEventRecord(p->ev[7], p->stream));
   CK(cudaStreamSynchronize(p->stream));
@@ -1323,7 +1242,7 @@ int icikt_plan_timings(icikt_plan* p, icikt_timings* t) {
     // pipelined call: kernel times are sums over the launches; h2d = start until the last column has landed,
     // d2h = first result copy until the last one (both overlap the kernels, so the parts exceed total_ms)
     for (size_t l = 0; l < p->stages.size(); ++l) {
-      const cudaEvent_t* e = &p->time_ev[5 * l];
+      const Event* e = &p->time_ev[5 * l];
       if (p->stages[l].col_hi > p->stages[l].col_lo) t->columns_ms += ev_ms(e[0], e[1]);
       t->pairs_ms += ev_ms(e[2], e[3]);
       t->epilogue_ms += ev_ms(e[3], e[4]);
@@ -1339,7 +1258,7 @@ int icikt_plan_timings(icikt_plan* p, icikt_timings* t) {
   return ICIKT_OK;
 }
 
-void icikt_plan_destroy(icikt_plan* p) { free_plan(p); }
+void icikt_plan_destroy(icikt_plan* p) { delete p; }
 
 // The pipelined one-shot call on a staged plan (build_stage_table): uploads on the copy stream chunk by chunk,
 // K1 of a chunk and the pair launches that need nothing beyond it on the compute stream, the results of
@@ -1353,8 +1272,8 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
   if (!s.csc() && (!s.data || s.ld < p->n)) return fail(ICIKT_ERR_BAD_ARG, "bad upload arguments");
   if (counts && !p->d_counts) return fail(ICIKT_ERR_BAD_ARG, "plan was created without want_counts");
   CK(cudaSetDevice(p->device));
-  if (!p->d_data_own) CK(dmalloc(&p->d_data_own, (size_t)p->n * p->C));
-  p->d_data = p->d_data_own;
+  CK(p->d_data_own.reserve((size_t)p->n * p->C));
+  p->d_data = p->d_data_own.get();
   p->ld = p->n;
   p->columns_done = false;
   p->pairs_done = false;
@@ -1366,7 +1285,7 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
   const size_t L = p->stages.size();
   for (size_t l = 0; l < L; ++l) {
     const StageLaunch& st = p->stages[l];
-    cudaEvent_t* te = &p->time_ev[5 * l];
+    const Event* te = &p->time_ev[5 * l];
     if (st.col_hi > st.col_lo) {
       int rc = copy_columns_in(p, s, st.col_lo, st.col_hi, p->copy_stream);
       if (rc != ICIKT_OK) return rc;
@@ -1376,7 +1295,7 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
       rc = plan_columns_impl(p, global_na, n_global_na, st.col_lo, st.col_hi, st.col_hi == p->C, st.col_lo == 0, te[0], te[1]);
       if (rc != ICIKT_OK) return rc;
     }
-    const int rc = launch_pair_group(p, p->d_units, st.unit_lo, st.unit_hi, st.max_unit_pairs, te[2], te[3], te[4], &pair_launches);
+    const int rc = launch_pair_group(p, p->d_units.get(), st.unit_lo, st.unit_hi, st.max_unit_pairs, te[2], te[3], te[4], &pair_launches);
     if (rc != ICIKT_OK) return rc;
     CK(cudaEventRecord(p->sync_ev[2 * l + 1], p->stream));
   }
@@ -1394,7 +1313,7 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
         {completeness, reinterpret_cast<const unsigned char*>(p->d_comp), sizeof(double), 3 * npad * sizeof(double)},
         {status, reinterpret_cast<const unsigned char*>(p->d_status), sizeof(int32_t),
          4 * npad * sizeof(double) + sizeof(unsigned long long)},
-        {counts, reinterpret_cast<const unsigned char*>(p->d_counts), sizeof(int64_t) * ICIKT_NCOUNTS, 0},
+        {counts, reinterpret_cast<const unsigned char*>(p->d_counts.get()), sizeof(int64_t) * ICIKT_NCOUNTS, 0},
     };
     if (p->h_res) {
       // every block's copies into the pinned mirror are enqueued at once (each waits for its block), the
@@ -1409,7 +1328,7 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
           if (!outs[k].host) continue;
           const size_t o = (size_t)st.slot_lo * outs[k].elem, b = (size_t)(st.slot_hi - st.slot_lo) * outs[k].elem;
           void* dst = (k == 5) ? static_cast<void*>(static_cast<unsigned char*>(outs[k].host) + o)
-                               : static_cast<void*>(p->h_res + outs[k].res_off + o);
+                               : static_cast<void*>(p->h_res.get() + outs[k].res_off + o);
           CK(cudaMemcpyAsync(dst, outs[k].dev + o, b, cudaMemcpyDeviceToHost, p->copy_stream));
         }
         CK(cudaEventRecord(p->sync_ev[2 * l], p->copy_stream));  // free since the block's columns were waited for
@@ -1421,7 +1340,7 @@ static int run_staged(icikt_plan* p, const ColumnSource& s, const double* global
         for (int k = 0; k < 5; ++k) {
           if (!outs[k].host) continue;
           const size_t o = (size_t)st.slot_lo * outs[k].elem, b = (size_t)(st.slot_hi - st.slot_lo) * outs[k].elem;
-          host_copy(static_cast<unsigned char*>(outs[k].host) + o, p->h_res + outs[k].res_off + o, b);
+          host_copy(static_cast<unsigned char*>(outs[k].host) + o, p->h_res.get() + outs[k].res_off + o, b);
         }
       }
     } else {
@@ -1657,33 +1576,26 @@ static int check_topk_args(const ColumnSource& s, int64_t n, int64_t C, const do
   return check_window_args(s, n, C, global_na, n_global_na, o);
 }
 
-#define ECK(call)                                                                                              \
-  do {                                                                                                         \
-    cudaError_t e_ = (call);                                                                                   \
-    if (e_ != cudaSuccess)                                                                                     \
-      return e_ == cudaErrorMemoryAllocation ? (cudaGetLastError(), fail(ICIKT_ERR_ALLOC, "allocation failed: " #call)) \
-                                             : cuda_fail(e_, #call);                                           \
-  } while (0)
 
 // the window walk's events, readbacks and staging chunks (kept with the plan)
 static int ensure_walk_buffers(icikt_plan* p) {
-  if (p->d_etotal) return ICIKT_OK;
-  if (!p->copy_stream) ECK(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
-  for (int b = 0; b < 2; ++b)
-    for (auto& e : p->eev[b]) ECK(cudaEventCreate(&e));
-  ECK(cudaMallocHost(reinterpret_cast<void**>(&p->h_estat), 4 * sizeof(unsigned long long)));
-  ECK(dmalloc(&p->d_etotal, 2));
+  if (!p->copy_stream) ECK(p->copy_stream.create());
+  for (auto& evs : p->eev)
+    for (Event& e : evs)
+      if (!e) ECK(e.create());
+  ECK(p->h_estat.reserve(4));
+  ECK(p->d_etotal.reserve(2));
   return ensure_stage(p);
 }
 
 // the edge selection's buffers for windows of W pairs (kept with the plan)
 static int ensure_edge_buffers(icikt_plan* p, int64_t W) {
   const int rc = ensure_walk_buffers(p);
-  if (rc != ICIKT_OK || p->d_erows[1]) return rc;
+  if (rc != ICIKT_OK) return rc;
   const int64_t tiles = (W + kEdgeTile - 1) / kEdgeTile;
-  ECK(dmalloc(&p->d_emask, (size_t)tiles * (kEdgeTile / 32)));
-  ECK(dmalloc(&p->d_etile, (size_t)tiles));
-  for (int b = 0; b < 2; ++b) ECK(dmalloc(&p->d_erows[b], (size_t)W));
+  ECK(p->d_emask.reserve((size_t)tiles * (kEdgeTile / 32)));
+  ECK(p->d_etile.reserve((size_t)tiles));
+  for (auto& rows : p->d_erows) ECK(rows.reserve((size_t)W));
   return ICIKT_OK;
 }
 
@@ -1692,63 +1604,33 @@ static int ensure_edge_buffers(icikt_plan* p, int64_t W) {
 static int ensure_topk_buffers(icikt_plan* p, int64_t W, int k, int64_t L) {
   const int rc = ensure_walk_buffers(p);
   if (rc != ICIKT_OK) return rc;
-  if (!p->d_tcand) ECK(dmalloc(&p->d_tcand, 2 * (size_t)W));
-  if (L > p->topk_cols) {
-    cudaFree(p->d_tcount);
-    cudaFree(p->d_tcol);
-    p->d_tcount = nullptr;
-    p->d_tcol = nullptr;
-    p->topk_cols = 0;
-    ECK(dmalloc(&p->d_tcount, (size_t)L));
-    ECK(dmalloc(&p->d_tcol, (size_t)L));
-    p->topk_cols = L;
-  }
-  if (L * k > p->topk_entries) {
-    cudaFree(p->d_tidx);
-    cudaFree(p->d_tlist);
-    p->d_tidx = nullptr;
-    p->d_tlist = nullptr;
-    p->topk_entries = 0;
-    ECK(dmalloc(&p->d_tidx, (size_t)(L * k)));
-    ECK(dmalloc(&p->d_tlist, 4 * (size_t)(L * k)));
-    p->topk_entries = L * k;
-  }
+  ECK(p->d_tcand.reserve(2 * (size_t)W));
+  ECK(p->d_tcount.reserve((size_t)L));
+  ECK(p->d_tcol.reserve((size_t)L));
+  ECK(p->d_tidx.reserve((size_t)(L * k)));
+  ECK(p->d_tlist.reserve(4 * (size_t)(L * k)));
   return ICIKT_OK;
 }
 
 // the merged lists of a block of columns (top-k over several devices): `entries` = columns of the block x k
 static int ensure_merge_buffers(icikt_plan* p, size_t entries) {
-  if (!p->d_mn) ECK(dmalloc(&p->d_mn, (size_t)p->C));
-  if (entries > p->merge_cap) {
-    cudaFree(p->d_midx);
-    cudaFree(p->d_mlist);
-    p->d_midx = nullptr;
-    p->d_mlist = nullptr;
-    p->merge_cap = 0;
-    ECK(dmalloc(&p->d_midx, entries));
-    ECK(dmalloc(&p->d_mlist, 4 * entries));
-    p->merge_cap = entries;
-  }
+  ECK(p->d_mn.reserve((size_t)p->C));
+  ECK(p->d_midx.reserve(entries));
+  ECK(p->d_mlist.reserve(4 * entries));
   return ensure_stage(p);
 }
 
 // room for `need` units in both window unit buffers (device and pinned host)
 static int ensure_window_units(icikt_plan* p, size_t need) {
-  if (need <= p->wunit_cap) return ICIKT_OK;
+  size_t have = p->d_wunits[0].size();
+  for (int b = 0; b < 2; ++b) have = std::min({have, p->d_wunits[b].size(), p->h_wunits[b].size()});
+  if (need <= have) return ICIKT_OK;
   CK(cudaStreamSynchronize(p->stream));  // the other buffer may still be read by the previous window
-  const size_t cap = std::max(need + need / 4, 2 * p->wunit_cap);
+  const size_t cap = std::max(need + need / 4, 2 * have);
   for (int b = 0; b < 2; ++b) {
-    cudaFree(p->d_wunits[b]);
-    if (p->h_wunits[b]) cudaFreeHost(p->h_wunits[b]);
-    p->d_wunits[b] = nullptr;
-    p->h_wunits[b] = nullptr;
+    ECK(p->d_wunits[b].reserve(cap));
+    ECK(p->h_wunits[b].reserve(cap));
   }
-  p->wunit_cap = 0;
-  for (int b = 0; b < 2; ++b) {
-    ECK(dmalloc(&p->d_wunits[b], cap));
-    ECK(cudaMallocHost(reinterpret_cast<void**>(&p->h_wunits[b]), sizeof(PairUnit) * cap));
-  }
-  p->wunit_cap = cap;
   return ICIKT_OK;
 }
 
@@ -1825,27 +1707,27 @@ static int walk_windows(icikt_plan* p, const Order& order, int64_t first, int64_
     int r = ensure_window_units(p, U.size());
     if (r != ICIKT_OK) return r;
     // the buffer was last read by window w - 2, whose selection the host has waited for
-    std::memcpy(p->h_wunits[b], U.data(), sizeof(PairUnit) * U.size());
+    std::memcpy(p->h_wunits[b].get(), U.data(), sizeof(PairUnit) * U.size());
     int max_unit = 1;
     for (const PairUnit& u : U) max_unit = std::max(max_unit, (int)u.count);
-    cudaEvent_t* e = p->eev[b];
+    const Event* e = p->eev[b];
     CK(cudaEventRecord(e[0], p->stream));
-    CK(cudaMemcpyAsync(p->d_wunits[b], p->h_wunits[b], sizeof(PairUnit) * U.size(), cudaMemcpyHostToDevice, p->stream));
+    CK(cudaMemcpyAsync(p->d_wunits[b].get(), p->h_wunits[b].get(), sizeof(PairUnit) * U.size(), cudaMemcpyHostToDevice, p->stream));
     CK(cudaEventRecord(e[1], p->stream));
-    r = launch_pair_group(p, p->d_wunits[b], 0, (int64_t)U.size(), max_unit, e[2], e[3], e[4], &tot.launches);
+    r = launch_pair_group(p, p->d_wunits[b].get(), 0, (int64_t)U.size(), max_unit, e[2], e[3], e[4], &tot.launches);
     if (r != ICIKT_OK) return r;
-    r = select(w, b, p->d_wunits[b], (int64_t)U.size(), hi - lo);
+    r = select(w, b, p->d_wunits[b].get(), (int64_t)U.size(), hi - lo);
     if (r != ICIKT_OK) return r;
-    CK(cudaMemcpyAsync(p->h_estat + 2 * b + 1, p->d_maxbits, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaMemcpyAsync(p->h_estat.get() + 2 * b + 1, p->d_maxbits, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
     CK(cudaEventRecord(e[5], p->stream));
     return ICIKT_OK;
   };
 
   auto wait = [&](int64_t w) -> int {
     const int b = (int)(w & 1);
-    cudaEvent_t* e = p->eev[b];
+    const Event* e = p->eev[b];
     CK(cudaEventSynchronize(e[5]));
-    tot.bits = p->h_estat[2 * b + 1];
+    tot.bits = p->h_estat.get()[2 * b + 1];
     tot.up_ms += ev_ms(e[0], e[1]);
     tot.pairs_ms += ev_ms(e[2], e[3]);
     tot.epi_ms += ev_ms(e[3], e[5]);
@@ -1884,26 +1766,15 @@ static int finish_walk(icikt_plan* p, const WalkTotals& tot, float d2h_ms, icikt
 // that holds every row whose adjusted value can pass).  The buffer grows geometrically; it always has room for the two
 // windows whose counts the host has not read back yet.
 struct PadjPart {
-  int device = -1;
-  unsigned long long* d_cnt = nullptr;   // [2]: non-NaN p-values, candidates
-  unsigned long long* h_cnt = nullptr;   // pinned [2][2]: the readback of d_cnt, per window buffer
-  unsigned long long* d_keys = nullptr;  // [cap]
-  int64_t cap = 0, known = 0;            // capacity; candidates as of the last readback
-  int64_t m = 0, K = 0;                  // after the walk: non-NaN p-values and candidates
-  double bound = 0.0;                    // the candidate bound (NaN: every non-NaN p-value)
-  PadjPart() = default;
-  PadjPart(const PadjPart&) = delete;
-  PadjPart& operator=(const PadjPart&) = delete;
-  ~PadjPart() { release(); }
-  void release() {
-    if (device < 0) return;
-    cudaSetDevice(device);
-    cudaFree(d_cnt);
-    cudaFree(d_keys);
-    if (h_cnt) cudaFreeHost(h_cnt);
-    d_cnt = d_keys = h_cnt = nullptr;
-    device = -1;
-    cap = 0;
+  int device = -1;                           // where the buffers live (-1: not set up)
+  DeviceArray<unsigned long long> d_cnt;     // [2]: non-NaN p-values, candidates
+  PinnedArray<unsigned long long> h_cnt;     // [2][2]: the readback of d_cnt, per window buffer
+  DeviceArray<unsigned long long> d_keys;    // its size is the capacity
+  int64_t known = 0;                         // candidates as of the last readback
+  int64_t m = 0, K = 0;                      // after the walk: non-NaN p-values and candidates
+  double bound = 0.0;                        // the candidate bound (NaN: every non-NaN p-value)
+  ~PadjPart() {
+    if (device >= 0) cudaSetDevice(device);
   }
 };
 
@@ -1911,33 +1782,29 @@ struct PadjPart {
 static int padj_room(icikt_plan* p, PadjPart& a, int64_t more) {
   if (a.device < 0) {
     a.device = p->device;
-    ECK(dmalloc(&a.d_cnt, 2));
-    ECK(cudaMallocHost(reinterpret_cast<void**>(&a.h_cnt), 4 * sizeof(unsigned long long)));
-    std::memset(a.h_cnt, 0, 4 * sizeof(unsigned long long));
-    CK(cudaMemsetAsync(a.d_cnt, 0, 2 * sizeof(unsigned long long), p->stream));
+    ECK(a.d_cnt.reserve(2));
+    ECK(a.h_cnt.reserve(4));
+    std::memset(a.h_cnt.get(), 0, 4 * sizeof(unsigned long long));
+    CK(cudaMemsetAsync(a.d_cnt.get(), 0, 2 * sizeof(unsigned long long), p->stream));
   }
-  if (a.known + more <= a.cap) return ICIKT_OK;
+  if (a.known + more <= (int64_t)a.d_keys.size()) return ICIKT_OK;
   CK(cudaStreamSynchronize(p->stream));  // the windows in flight append to the old buffer
   unsigned long long now[2];
-  CK(cudaMemcpy(now, a.d_cnt, sizeof(now), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(now, a.d_cnt.get(), sizeof(now), cudaMemcpyDeviceToHost));
   a.known = (int64_t)now[1];
-  const int64_t cap = std::max(2 * a.cap, a.known + more);
-  unsigned long long* keys = nullptr;
-  if (dmalloc(&keys, (size_t)cap) != cudaSuccess) {
+  const int64_t cap = std::max(2 * (int64_t)a.d_keys.size(), a.known + more);
+  DeviceArray<unsigned long long> keys;
+  if (keys.reserve((size_t)cap) != cudaSuccess) {
     cudaGetLastError();
     return fail(ICIKT_ERR_ALLOC, "device allocation for " + std::to_string(cap) + " p-value candidates failed (" +
                                      std::to_string(a.known) + " held)");
   }
   if (a.known) {
-    const cudaError_t e = cudaMemcpy(keys, a.d_keys, sizeof(unsigned long long) * (size_t)a.known, cudaMemcpyDeviceToDevice);
-    if (e != cudaSuccess) {
-      cudaFree(keys);
-      return cuda_fail(e, "p-value candidates");
-    }
+    const cudaError_t e = cudaMemcpy(keys.get(), a.d_keys.get(), sizeof(unsigned long long) * (size_t)a.known,
+                                     cudaMemcpyDeviceToDevice);
+    if (e != cudaSuccess) return cuda_fail(e, "p-value candidates");
   }
-  cudaFree(a.d_keys);
-  a.d_keys = keys;
-  a.cap = cap;
+  a.d_keys = std::move(keys);
   return ICIKT_OK;
 }
 
@@ -1982,28 +1849,28 @@ static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter&
     es.min_abs_cor = f.min_abs_cor;
     es.max_pvalue = f.max_pvalue;
     es.scale_max = scale ? 1 : 0;
-    es.mask = p->d_emask;
-    es.tile_offset = p->d_etile;
-    es.total = p->d_etotal + b;
-    es.rows = p->d_erows[b];
+    es.mask = p->d_emask.get();
+    es.tile_offset = p->d_etile.get();
+    es.total = p->d_etotal.get() + b;
+    es.rows = p->d_erows[b].get();
     const int l = launch_edge_select(es, p->stream);
     if (l < 0) return launch_fail("edge selection kernels");
     tot.launches += l;
-    CK(cudaMemcpyAsync(p->h_estat + 2 * b, p->d_etotal + b, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaMemcpyAsync(p->h_estat.get() + 2 * b, p->d_etotal.get() + b, sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
     if (adj) {  // the window's non-NaN count and candidates, in the epilogue's time
       const int r = padj_room(p, *adj, 2 * W);
       if (r != ICIKT_OK) return r;
-      CK(padj_candidates(p->d_p, n_slots, adj->bound, adj->d_cnt, adj->d_keys, p->stream));
-      CK(cudaMemcpyAsync(adj->h_cnt + 2 * b, adj->d_cnt, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
+      CK(padj_candidates(p->d_p, n_slots, adj->bound, adj->d_cnt.get(), adj->d_keys.get(), p->stream));
+      CK(cudaMemcpyAsync(adj->h_cnt.get() + 2 * b, adj->d_cnt.get(), 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, p->stream));
     }
     return ICIKT_OK;
   };
 
   auto collect = [&](int64_t w, int b) -> int {
     if (held.stop) return edge_limit_fail(f, held.total, " held when another device reached the limit");
-    const unsigned long long cnt = p->h_estat[2 * b];
+    const unsigned long long cnt = p->h_estat.get()[2 * b];
     const unsigned long long bits = tot.bits;
-    if (adj) adj->known = std::max<int64_t>(adj->known, (int64_t)adj->h_cnt[2 * b + 1]);
+    if (adj) adj->known = std::max<int64_t>(adj->known, (int64_t)adj->h_cnt.get()[2 * b + 1]);
     const size_t before = rows.size();
     if (cnt) {
       const size_t old = rows.size();
@@ -2013,7 +1880,7 @@ static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter&
         return fail(ICIKT_ERR_ALLOC, "out of host memory for the selected rows");
       }
       CK(cudaEventRecord(p->ev[6], p->copy_stream));
-      const int r = staged_copy_out(p, rows.data() + old, p->d_erows[b], sizeof(EdgeRow) * (size_t)cnt, p->copy_stream);
+      const int r = staged_copy_out(p, rows.data() + old, p->d_erows[b].get(), sizeof(EdgeRow) * (size_t)cnt, p->copy_stream);
       if (r != ICIKT_OK) return r;
       CK(cudaEventRecord(p->ev[7], p->copy_stream));
       CK(cudaEventSynchronize(p->ev[7]));
@@ -2037,7 +1904,7 @@ static int edge_walk(icikt_plan* p, const Order& order, const icikt_edge_filter&
   if (rc != ICIKT_OK || !adj || adj->device < 0) return rc;
   unsigned long long now[2];
   CK(cudaStreamSynchronize(p->stream));
-  CK(cudaMemcpy(now, adj->d_cnt, sizeof(now), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(now, adj->d_cnt.get(), sizeof(now), cudaMemcpyDeviceToHost));
   adj->m = (int64_t)now[0];
   adj->K = (int64_t)now[1];
   return ICIKT_OK;
@@ -2083,7 +1950,7 @@ template <class Order>
 static int topk_walk(icikt_plan* p, const Order& order, int64_t c_lo, int64_t c_hi, int k, int by, int64_t first,
                      int64_t last, int64_t W, WalkTotals& tot) {
   const int64_t ck = (c_hi - c_lo) * k;
-  CK(cudaMemsetAsync(p->d_tcol, 0, sizeof(TopkCol) * (size_t)(c_hi - c_lo), p->stream));
+  CK(cudaMemsetAsync(p->d_tcol.get(), 0, sizeof(TopkCol) * (size_t)(c_hi - c_lo), p->stream));
   auto select = [&](int64_t, int b, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
     TopkSelect ts;
     ts.units = units;
@@ -2098,15 +1965,15 @@ static int topk_walk(icikt_plan* p, const Order& order, int64_t c_lo, int64_t c_
     ts.c_hi = c_hi;
     ts.k = k;
     ts.by = by;
-    ts.col_count = p->d_tcount;
-    ts.total = p->d_etotal + b;
-    ts.cand = p->d_tcand;
-    ts.col = p->d_tcol;
-    ts.idx = p->d_tidx;
-    ts.raw = p->d_tlist;
-    ts.pv = p->d_tlist + ck;
-    ts.tm = p->d_tlist + 2 * ck;
-    ts.comp = p->d_tlist + 3 * ck;
+    ts.col_count = p->d_tcount.get();
+    ts.total = p->d_etotal.get() + b;
+    ts.cand = p->d_tcand.get();
+    ts.col = p->d_tcol.get();
+    ts.idx = p->d_tidx.get();
+    ts.raw = p->d_tlist.get();
+    ts.pv = p->d_tlist.get() + ck;
+    ts.tm = p->d_tlist.get() + 2 * ck;
+    ts.comp = p->d_tlist.get() + 3 * ck;
     const int l = launch_topk_select(ts, p->stream);
     if (l < 0) return launch_fail("top-k selection kernels");
     tot.launches += l;
@@ -2169,8 +2036,6 @@ static void topk_sides_finish(std::vector<TopkSide>& sides, int k, Held&& held, 
     topk_fill_host(sd.out, sd.cols, k, side_held, sd.raw, scale, M);
   }
 }
-
-#undef ECK
 
 extern "C" {
 
@@ -2249,8 +2114,8 @@ static int ensure_cross_buffers(icikt_plan* p) {
   const int rc = ensure_walk_buffers(p);
   if (rc != ICIKT_OK) return rc;
   const size_t win = (size_t)p->P;  // the plan's pair buffers: W pairs and more
-  for (int b = 0; b < 2; ++b)
-    if (!p->d_cres[b] && cudaMalloc(reinterpret_cast<void**>(&p->d_cres[b]), win * (4 * sizeof(double) + sizeof(int32_t))) != cudaSuccess) {
+  for (auto& res : p->d_cres)
+    if (res.reserve(win * (4 * sizeof(double) + sizeof(int32_t))) != cudaSuccess) {
       cudaGetLastError();
       return fail(ICIKT_ERR_ALLOC, "device allocation of the cross call's result windows failed");
     }
@@ -2268,7 +2133,7 @@ static int cross_pair_walk(icikt_plan* p, int64_t Cx, int64_t Cy, int64_t first,
   const double* d_field[4] = {p->d_tau, p->d_p, p->d_tm, p->d_comp};
   double* host_field[4] = {raw, pvalue, taumax, completeness};
   auto select = [&](int64_t, int b, const PairUnit*, int64_t, int64_t n_slots) -> int {
-    double* to = reinterpret_cast<double*>(p->d_cres[b]);
+    double* to = reinterpret_cast<double*>(p->d_cres[b].get());
     for (int f = 0; f < 4; ++f)
       if (host_field[f])
         CK(cudaMemcpyAsync(to + f * win, d_field[f], sizeof(double) * (size_t)n_slots, cudaMemcpyDeviceToDevice, p->stream));
@@ -2278,7 +2143,7 @@ static int cross_pair_walk(icikt_plan* p, int64_t Cx, int64_t Cy, int64_t first,
   };
   auto collect = [&](int64_t w, int b) -> int {
     const int64_t off = w * W, cnt = std::min(W, last - first - off);
-    const double* from = reinterpret_cast<const double*>(p->d_cres[b]);
+    const double* from = reinterpret_cast<const double*>(p->d_cres[b].get());
     CK(cudaEventRecord(p->ev[6], p->copy_stream));
     int r = ICIKT_OK;
     for (int f = 0; f < 4 && r == ICIKT_OK; ++f)
@@ -2335,61 +2200,57 @@ static int pairwise_completeness_impl(const ColumnSource& s, int64_t n, int64_t 
   const int64_t words = (n + 31) / 32;
   const bool per_pair = missing || completeness;
   struct Buffers {
-    double *data = nullptr, *lit = nullptr, *comp = nullptr, *mat = nullptr, *values = nullptr;
-    uint32_t* bits = nullptr;
-    int32_t *pi = nullptr, *pj = nullptr, *miss = nullptr, *rowidx = nullptr;
-    int64_t* colptr = nullptr;
-    cudaStream_t stream = nullptr;
+    Stream stream;  // released after the buffers
+    DeviceArray<double> data, lit, comp, mat, values;
+    DeviceArray<uint32_t> bits;
+    DeviceArray<int32_t> pi, pj, miss, rowidx;
+    DeviceArray<int64_t> colptr;
     ~Buffers() {
       if (stream) cudaStreamSynchronize(stream);  // no copy still reads the caller's arrays after an error
-      cudaFree(data); cudaFree(lit); cudaFree(comp); cudaFree(mat); cudaFree(bits);
-      cudaFree(pi); cudaFree(pj); cudaFree(miss);
-      cudaFree(colptr); cudaFree(rowidx); cudaFree(values);
-      if (stream) cudaStreamDestroy(stream);
     }
   } b;
-  CK(cudaStreamCreateWithFlags(&b.stream, cudaStreamNonBlocking));
-  CK(dmalloc(&b.data, (size_t)n * C));
-  CK(dmalloc(&b.lit, 64));
-  CK(dmalloc(&b.bits, (size_t)words * C));
+  CK(b.stream.create());
+  CK(b.data.reserve((size_t)n * C));
+  CK(b.lit.reserve(64));
+  CK(b.bits.reserve((size_t)words * C));
   if (s.csc()) {  // the stored entries, expanded into the dense matrix on the device
     const int64_t nnz = s.colptr[C];
-    CK(dmalloc(&b.colptr, (size_t)C + 1));
-    CK(dmalloc(&b.rowidx, (size_t)nnz));
-    CK(dmalloc(&b.values, (size_t)nnz));
-    CK(cudaMemcpyAsync(b.colptr, s.colptr, sizeof(int64_t) * (size_t)(C + 1), cudaMemcpyHostToDevice, b.stream));
+    CK(b.colptr.reserve((size_t)C + 1));
+    CK(b.rowidx.reserve((size_t)nnz));
+    CK(b.values.reserve((size_t)nnz));
+    CK(cudaMemcpyAsync(b.colptr.get(), s.colptr, sizeof(int64_t) * (size_t)(C + 1), cudaMemcpyHostToDevice, b.stream));
     if (nnz) {
-      CK(cudaMemcpyAsync(b.rowidx, s.rowidx, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, b.stream));
-      CK(cudaMemcpyAsync(b.values, s.values, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, b.stream));
+      CK(cudaMemcpyAsync(b.rowidx.get(), s.rowidx, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, b.stream));
+      CK(cudaMemcpyAsync(b.values.get(), s.values, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, b.stream));
     }
-    if (launch_csc_expand(b.colptr, b.rowidx, b.values, n, 0, C, b.data, b.stream) < 0)
+    if (launch_csc_expand(b.colptr.get(), b.rowidx.get(), b.values.get(), n, 0, C, b.data.get(), b.stream) < 0)
       return launch_fail("CSC expansion kernel");
   } else {
-    CK(cudaMemcpy2DAsync(b.data, sizeof(double) * n, s.data, sizeof(double) * s.ld, sizeof(double) * n, (size_t)C,
+    CK(cudaMemcpy2DAsync(b.data.get(), sizeof(double) * n, s.data, sizeof(double) * s.ld, sizeof(double) * n, (size_t)C,
                          cudaMemcpyHostToDevice, b.stream));
   }
-  if (nlit) CK(cudaMemcpyAsync(b.lit, lit, sizeof(double) * nlit, cudaMemcpyHostToDevice, b.stream));
-  if (launch_missing_bits(b.data, n, n, C, b.lit, nlit, na_nan, na_inf, b.bits, words, b.stream) < 0)
+  if (nlit) CK(cudaMemcpyAsync(b.lit.get(), lit, sizeof(double) * nlit, cudaMemcpyHostToDevice, b.stream));
+  if (launch_missing_bits(b.data.get(), n, n, C, b.lit.get(), nlit, na_nan, na_inf, b.bits.get(), words, b.stream) < 0)
     return launch_fail("missing-mask kernel");
   if (per_pair) {
     if (pi) {
-      CK(dmalloc(&b.pi, (size_t)P));
-      CK(dmalloc(&b.pj, (size_t)P));
-      CK(cudaMemcpyAsync(b.pi, pi, sizeof(int32_t) * P, cudaMemcpyHostToDevice, b.stream));
-      CK(cudaMemcpyAsync(b.pj, pj, sizeof(int32_t) * P, cudaMemcpyHostToDevice, b.stream));
+      CK(b.pi.reserve((size_t)P));
+      CK(b.pj.reserve((size_t)P));
+      CK(cudaMemcpyAsync(b.pi.get(), pi, sizeof(int32_t) * P, cudaMemcpyHostToDevice, b.stream));
+      CK(cudaMemcpyAsync(b.pj.get(), pj, sizeof(int32_t) * P, cudaMemcpyHostToDevice, b.stream));
     }
-    if (missing) CK(dmalloc(&b.miss, (size_t)P));
-    if (completeness) CK(dmalloc(&b.comp, (size_t)P));
-    if (launch_pair_missing(b.bits, words, n, C, b.pi, b.pj, P, b.miss, b.comp, b.stream) < 0)
+    if (missing) CK(b.miss.reserve((size_t)P));
+    if (completeness) CK(b.comp.reserve((size_t)P));
+    if (launch_pair_missing(b.bits.get(), words, n, C, b.pi.get(), b.pj.get(), P, b.miss.get(), b.comp.get(), b.stream) < 0)
       return launch_fail("pair completeness kernel");
-    if (missing) CK(cudaMemcpyAsync(missing, b.miss, sizeof(int32_t) * P, cudaMemcpyDeviceToHost, b.stream));
-    if (completeness) CK(cudaMemcpyAsync(completeness, b.comp, sizeof(double) * P, cudaMemcpyDeviceToHost, b.stream));
+    if (missing) CK(cudaMemcpyAsync(missing, b.miss.get(), sizeof(int32_t) * P, cudaMemcpyDeviceToHost, b.stream));
+    if (completeness) CK(cudaMemcpyAsync(completeness, b.comp.get(), sizeof(double) * P, cudaMemcpyDeviceToHost, b.stream));
   }
   if (matrix) {
-    CK(dmalloc(&b.mat, (size_t)C * C));
-    if (launch_missing_matrix(b.bits, words, n, C, b.mat, b.stream) < 0)
+    CK(b.mat.reserve((size_t)C * C));
+    if (launch_missing_matrix(b.bits.get(), words, n, C, b.mat.get(), b.stream) < 0)
       return launch_fail("completeness matrix kernel");
-    CK(cudaMemcpyAsync(matrix, b.mat, sizeof(double) * C * C, cudaMemcpyDeviceToHost, b.stream));
+    CK(cudaMemcpyAsync(matrix, b.mat.get(), sizeof(double) * C * C, cudaMemcpyDeviceToHost, b.stream));
   }
   CK(cudaStreamSynchronize(b.stream));
   return ICIKT_OK;
@@ -2721,24 +2582,11 @@ int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* glo
       const int64_t c_lo = J.col_lo(k), c_hi = J.col_lo(k + 1);
       const size_t blk = (size_t)C * (size_t)(c_hi - c_lo);
       CK(cudaSetDevice(p->device));
-      if (p->mat_elems < 5 * blk) {
-        cudaFree(p->d_mat);
-        p->d_mat = nullptr;
-        p->mat_elems = 0;
-        if (dmalloc(&p->d_mat, 5 * blk) != cudaSuccess) {
-          cudaGetLastError();
-          return fail(ICIKT_ERR_ALLOC, "device allocation of the result matrix block failed");
-        }
-        p->mat_elems = 5 * blk;
-      }
-      if (!p->d_hist) CK(dmalloc(&p->d_hist, 16));
-      if (!p->d_ngood) CK(dmalloc(&p->d_ngood, (size_t)C));
-      {
-        const int r3 = ensure_stage(p);
-        if (r3 != ICIKT_OK) return r3;
-      }
+      int r = ensure_matrix_buffers(p, 5 * blk, "the result matrix block");
+      if (r == ICIKT_OK) r = ensure_stage(p);
+      if (r != ICIKT_OK) return r;
       CK(cudaEventRecord(p->ev[6], p->stream));
-      CK(cudaMemsetAsync(p->d_hist, 0, 16 * sizeof(unsigned long long), p->stream));
+      CK(cudaMemsetAsync(p->d_hist.get(), 0, 16 * sizeof(unsigned long long), p->stream));
       BlockFill f{};
       f.n_dev = n_dev;
       for (int j = 0; j < n_dev; ++j) {
@@ -2751,23 +2599,23 @@ int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* glo
       f.n = n; f.C = C; f.c_lo = c_lo; f.c_hi = c_hi;
       f.scale_max = scale_max != 0; f.diag_good = diag_good != 0;
       f.max_taumax = mx;
-      f.n_good = p->d_ngood;
+      f.n_good = p->d_ngood.get();
       int best = 1;
       if (diag_good) {
-        CK(cudaMemcpyAsync(p->d_ngood, good.data(), sizeof(int32_t) * (size_t)C, cudaMemcpyHostToDevice, p->stream));
+        CK(cudaMemcpyAsync(p->d_ngood.get(), good.data(), sizeof(int32_t) * (size_t)C, cudaMemcpyHostToDevice, p->stream));
         best = 0;
         for (int64_t c = 0; c < C; ++c) best = std::max(best, good[(size_t)c]);
       }
       f.best_good = best;
-      for (int q = 0; q < 5; ++q) f.m[q] = outs[q] ? p->d_mat + (size_t)q * blk : nullptr;
-      f.hist = p->d_hist;
+      for (int q = 0; q < 5; ++q) f.m[q] = outs[q] ? p->d_mat.get() + (size_t)q * blk : nullptr;
+      f.hist = p->d_hist.get();
       if (launch_matrix_block_fill(f, p->stream) < 0) return launch_fail("matrix block fill kernel");
       for (int q = 0; q < 5; ++q)
         if (outs[q] && blk) {
           const int r2 = staged_copy_out(p, outs[q] + (size_t)c_lo * (size_t)C, f.m[q], sizeof(double) * blk, p->stream);
           if (r2 != ICIKT_OK) return r2;
         }
-      CK(cudaMemcpyAsync(w.hist, p->d_hist, sizeof(w.hist), cudaMemcpyDeviceToHost, p->stream));
+      CK(cudaMemcpyAsync(w.hist, p->d_hist.get(), sizeof(w.hist), cudaMemcpyDeviceToHost, p->stream));
       CK(cudaEventRecord(p->ev[7], p->stream));
       CK(cudaStreamSynchronize(p->stream));
       return icikt_plan_timings(p, &w.tm);
@@ -2838,24 +2686,23 @@ int no_pairs(double* max_taumax, icikt_timings* timings) {
 // access between all devices: peer copies; otherwise through pinned host memory), sorted and scanned there once, and
 // every row looks its value up there.  m <= 1 leaves the p-values as they are (p.adjust).  Then the rows with
 // padj > max_padj go.  dev_ms receives the device time of the gather, sort, scan and lookup.
-using DevPtr = std::unique_ptr<void, cudaError_t (*)(void*)>;
-
-int padj_gather(const MultiJob& J, std::vector<PadjPart>& parts, int dev, int64_t K, unsigned long long** all, DevPtr& own) {
+int padj_gather(const MultiJob& J, std::vector<PadjPart>& parts, int dev, int64_t K, unsigned long long** all,
+                DeviceArray<unsigned long long>& own) {
   PadjPart& first = parts[0];
   int64_t at = 0;
   size_t k0 = 0;
-  if (first.device == dev && first.cap >= K) {  // the first worker's buffer takes the others' candidates
-    *all = first.d_keys;
+  if (first.device == dev && (int64_t)first.d_keys.size() >= K) {  // the first worker's buffer takes the others' candidates
+    *all = first.d_keys.get();
     at = first.K;
     k0 = 1;
   } else {
-    if (dmalloc(all, (size_t)K) != cudaSuccess) {
+    if (own.reserve((size_t)K) != cudaSuccess) {
       cudaGetLastError();
       return fail(ICIKT_ERR_ALLOC, "device allocation for the " + std::to_string(K) + " p-value candidates failed");
     }
-    own.reset(*all);
+    *all = own.get();
   }
-  unsigned long long* stage = nullptr;
+  PinnedArray<unsigned long long> stage;
   const size_t chunk = 4u << 20;  // keys per staged piece (32 MB)
   int rc = ICIKT_OK;
   for (size_t k = k0; k < parts.size() && rc == ICIKT_OK; ++k) {
@@ -2864,26 +2711,27 @@ int padj_gather(const MultiJob& J, std::vector<PadjPart>& parts, int dev, int64_
     cudaError_t e = cudaSuccess;
     if (!pt.K) continue;
     if (pt.device == dev) {
-      e = cudaMemcpy(*all + at, pt.d_keys, bytes, cudaMemcpyDeviceToDevice);
+      e = cudaMemcpy(*all + at, pt.d_keys.get(), bytes, cudaMemcpyDeviceToDevice);
     } else if (J.peers_ok) {
-      e = cudaMemcpyPeer(*all + at, dev, pt.d_keys, pt.device, bytes);
+      e = cudaMemcpyPeer(*all + at, dev, pt.d_keys.get(), pt.device, bytes);
     } else {
-      if (!stage && (e = cudaMallocHost(reinterpret_cast<void**>(&stage), sizeof(unsigned long long) * chunk)) != cudaSuccess)
-        break;
+      if ((e = stage.reserve(chunk)) != cudaSuccess) break;
       for (int64_t o = 0; o < pt.K && e == cudaSuccess; o += (int64_t)chunk) {
         const size_t b = sizeof(unsigned long long) * std::min<size_t>(chunk, (size_t)(pt.K - o));
-        if ((e = cudaSetDevice(pt.device)) == cudaSuccess) e = cudaMemcpy(stage, pt.d_keys + o, b, cudaMemcpyDeviceToHost);
+        if ((e = cudaSetDevice(pt.device)) == cudaSuccess) e = cudaMemcpy(stage.get(), pt.d_keys.get() + o, b, cudaMemcpyDeviceToHost);
         if (e == cudaSuccess && (e = cudaSetDevice(dev)) == cudaSuccess)
-          e = cudaMemcpy(*all + at + o, stage, b, cudaMemcpyHostToDevice);
+          e = cudaMemcpy(*all + at + o, stage.get(), b, cudaMemcpyHostToDevice);
       }
-      cudaSetDevice(dev);
     }
     if (e != cudaSuccess) rc = cuda_fail(e, "gathering the p-value candidates");
     at += pt.K;
-    pt.release();
+    cudaSetDevice(pt.device);  // the part is gathered: free its buffers on their device now
+    pt.d_keys.reset();
+    pt.d_cnt.reset();
+    pt.h_cnt.reset();
+    pt.device = -1;
     cudaSetDevice(dev);
   }
-  if (stage) cudaFreeHost(stage);
   return rc;
 }
 
@@ -2909,25 +2757,23 @@ int padj_finish(const MultiJob& J, std::vector<PadjPart>& parts, const icikt_pad
   } else if (R > 0) {
     const int dev = J.device_of(0);
     CK(cudaSetDevice(dev));
-    cudaEvent_t ev[2] = {nullptr, nullptr};
-    CK(cudaEventCreate(&ev[0]));
-    std::unique_ptr<CUevent_st, cudaError_t (*)(cudaEvent_t)> e0(ev[0], cudaEventDestroy);
-    CK(cudaEventCreate(&ev[1]));
-    std::unique_ptr<CUevent_st, cudaError_t (*)(cudaEvent_t)> e1(ev[1], cudaEventDestroy);
+    Event ev[2];
+    CK(ev[0].create());
+    CK(ev[1].create());
     CK(cudaEventRecord(ev[0], 0));
     unsigned long long* all = nullptr;
-    DevPtr own(nullptr, cudaFree);
+    DeviceArray<unsigned long long> own;
     int rc = padj_gather(J, parts, dev, K, &all, own);
     if (rc != ICIKT_OK) return rc;
     const double q = a.method == ICIKT_PADJ_BY ? padj_by_q(m) : 0.0;
-    unsigned long long *alt = nullptr, *sorted = nullptr;
-    double *vals = nullptr, *d_p = nullptr;
-    if (dmalloc(&alt, (size_t)K) != cudaSuccess || dmalloc(&d_p, 2 * (size_t)R) != cudaSuccess) {
+    unsigned long long* sorted = nullptr;
+    double* vals = nullptr;
+    DeviceArray<unsigned long long> alt;
+    DeviceArray<double> d_p;
+    if (alt.reserve((size_t)K) != cudaSuccess || d_p.reserve(2 * (size_t)R) != cudaSuccess) {
       cudaGetLastError();
-      cudaFree(alt);
       return fail(ICIKT_ERR_ALLOC, "device allocation for sorting " + std::to_string(K) + " p-value candidates failed");
     }
-    DevPtr own_alt(alt, cudaFree), own_p(d_p, cudaFree);
     std::vector<double> p;
     try {
       p.resize((size_t)R);
@@ -2935,10 +2781,10 @@ int padj_finish(const MultiJob& J, std::vector<PadjPart>& parts, const icikt_pad
       return fail(ICIKT_ERR_ALLOC, "out of host memory for the adjusted p-values");
     }
     for (int64_t r = 0; r < R; ++r) p[(size_t)r] = rows[(size_t)r].pvalue;
-    CK(padj_sort_scan(all, alt, K, m, a.method, q, &sorted, &vals, 0));
-    CK(cudaMemcpy(d_p, p.data(), sizeof(double) * (size_t)R, cudaMemcpyHostToDevice));
-    CK(padj_lookup(sorted, vals, K, a.method, d_p, R, d_p + R, 0));
-    CK(cudaMemcpy(padj.data(), d_p + R, sizeof(double) * (size_t)R, cudaMemcpyDeviceToHost));
+    CK(padj_sort_scan(all, alt.get(), K, m, a.method, q, &sorted, &vals, 0));
+    CK(cudaMemcpy(d_p.get(), p.data(), sizeof(double) * (size_t)R, cudaMemcpyHostToDevice));
+    CK(padj_lookup(sorted, vals, K, a.method, d_p.get(), R, d_p.get() + R, 0));
+    CK(cudaMemcpy(padj.data(), d_p.get() + R, sizeof(double) * (size_t)R, cudaMemcpyDeviceToHost));
     CK(cudaEventRecord(ev[1], 0));
     CK(cudaEventSynchronize(ev[1]));
     *dev_ms = ev_ms(ev[0], ev[1]);
@@ -3056,15 +2902,15 @@ int topk_copy_lists(icikt_plan* p, int64_t L, int K, const std::vector<TopkSide>
     return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
   }
   CK(cudaEventRecord(p->ev[6], p->stream));
-  int rc = staged_copy_out(p, col.data(), p->d_tcol, sizeof(TopkCol) * (size_t)L, p->stream);
+  int rc = staged_copy_out(p, col.data(), p->d_tcol.get(), sizeof(TopkCol) * (size_t)L, p->stream);
   const int64_t lk = L * K;
   for (const TopkSide& sd : sides) {
     const int64_t ck = sd.cols * K, at = sd.row0 * K;
-    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index, p->d_tidx + at, sizeof(int32_t) * (size_t)ck, p->stream);
+    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index, p->d_tidx.get() + at, sizeof(int32_t) * (size_t)ck, p->stream);
     double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
     for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
       if (host_field[f])
-        rc = staged_copy_out(p, host_field[f], p->d_tlist + f * lk + at, sizeof(double) * (size_t)ck, p->stream);
+        rc = staged_copy_out(p, host_field[f], p->d_tlist.get() + f * lk + at, sizeof(double) * (size_t)ck, p->stream);
   }
   if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[7], p->stream));
@@ -3088,33 +2934,33 @@ int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<
   TopkDeviceMerge m{};
   m.n_dev = J.n_devices;
   for (int j = 0; j < J.n_devices; ++j) {
-    m.col[j] = plans[(size_t)j]->d_tcol;
-    m.idx[j] = plans[(size_t)j]->d_tidx;
-    m.list[j] = plans[(size_t)j]->d_tlist;
+    m.col[j] = plans[(size_t)j]->d_tcol.get();
+    m.idx[j] = plans[(size_t)j]->d_tidx.get();
+    m.list[j] = plans[(size_t)j]->d_tlist.get();
   }
   m.C = L;  // the lists' rows: the kernel's columns
   m.c_lo = r_lo;
   m.c_hi = r_hi;
   m.k = K;
   m.by = by;
-  m.n = p->d_mn;
-  m.out_idx = p->d_midx;
-  m.out = p->d_mlist;
+  m.n = p->d_mn.get();
+  m.out_idx = p->d_midx.get();
+  m.out = p->d_mlist.get();
   CK(cudaEventRecord(p->ev[6], p->stream));
   const int l = launch_topk_device_merge(m, p->stream);
   if (l < 0) return launch_fail("top-k device merge kernel");
   tm.n_launches += l;
-  rc = staged_copy_out(p, held + r_lo, p->d_mn, sizeof(int32_t) * (size_t)(r_hi - r_lo), p->stream);
+  rc = staged_copy_out(p, held + r_lo, p->d_mn.get(), sizeof(int32_t) * (size_t)(r_hi - r_lo), p->stream);
   for (const TopkSide& sd : sides) {
     const int64_t lo = std::max(r_lo, sd.row0), hi = std::min(r_hi, sd.row0 + sd.cols);
     if (hi <= lo) continue;
     const size_t len = (size_t)(hi - lo) * (size_t)K, from = (size_t)(lo - r_lo) * (size_t)K,
                  to = (size_t)(lo - sd.row0) * (size_t)K;
-    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index + to, p->d_midx + from, sizeof(int32_t) * len, p->stream);
+    if (rc == ICIKT_OK) rc = staged_copy_out(p, sd.out.index + to, p->d_midx.get() + from, sizeof(int32_t) * len, p->stream);
     double* host_field[4] = {sd.raw, sd.out.pvalue, sd.out.taumax, sd.out.completeness};
     for (int f = 0; f < 4 && rc == ICIKT_OK; ++f)
       if (host_field[f])
-        rc = staged_copy_out(p, host_field[f] + to, p->d_mlist + f * blk + from, sizeof(double) * len, p->stream);
+        rc = staged_copy_out(p, host_field[f] + to, p->d_mlist.get() + f * blk + from, sizeof(double) * len, p->stream);
   }
   if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[7], p->stream));
@@ -3618,15 +3464,13 @@ int icikt_pnorm_device(const double* z, int64_t n, int32_t lower_tail, double* o
   int rc = select_device(device);
   if (rc != ICIKT_OK) return rc;
   if (n == 0) return ICIKT_OK;
-  double *dz = nullptr, *dout = nullptr;
-  CK(dmalloc(&dz, (size_t)n));
-  cudaError_t e = dmalloc(&dout, (size_t)n);
-  if (e != cudaSuccess) { cudaFree(dz); return cuda_fail(e, "cudaMalloc"); }
-  e = cudaMemcpy(dz, z, sizeof(double) * n, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = (launch_pnorm(dz, n, lower_tail, dout, 0) < 0) ? cudaGetLastError() : cudaSuccess;
-  if (e == cudaSuccess) e = cudaMemcpy(out, dout, sizeof(double) * n, cudaMemcpyDeviceToHost);
-  cudaFree(dz);
-  cudaFree(dout);
+  DeviceArray<double> dz, dout;
+  CK(dz.reserve((size_t)n));
+  cudaError_t e = dout.reserve((size_t)n);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc");
+  e = cudaMemcpy(dz.get(), z, sizeof(double) * n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = (launch_pnorm(dz.get(), n, lower_tail, dout.get(), 0) < 0) ? cudaGetLastError() : cudaSuccess;
+  if (e == cudaSuccess) e = cudaMemcpy(out, dout.get(), sizeof(double) * n, cudaMemcpyDeviceToHost);
   if (e != cudaSuccess) return cuda_fail(e, "pnorm");
   return ICIKT_OK;
 }
@@ -3682,15 +3526,15 @@ int icikt_p_adjust(const double* p, int64_t m, int32_t method, int32_t device, d
   if (rc != ICIKT_OK) return rc;
   int64_t mm = 0;
   if (m > 0) {
-    double* d = nullptr;
-    if (dmalloc(&d, 2 * (size_t)m) != cudaSuccess) {
+    DeviceArray<double> d;
+    if (d.reserve(2 * (size_t)m) != cudaSuccess) {
       cudaGetLastError();
       return fail(ICIKT_ERR_ALLOC, "device allocation for " + std::to_string(m) + " p-values failed");
     }
-    cudaError_t e = cudaMemcpy(d, p, sizeof(double) * (size_t)m, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = padj_array(d, m, method, d + m, &mm, nullptr, 0);
-    if (e == cudaSuccess) e = cudaMemcpy(out, d + m, sizeof(double) * (size_t)m, cudaMemcpyDeviceToHost);
-    cudaFree(d);
+    cudaError_t e = cudaMemcpy(d.get(), p, sizeof(double) * (size_t)m, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = padj_array(d.get(), m, method, d.get() + m, &mm, nullptr, 0);
+    if (e == cudaSuccess) e = cudaMemcpy(out, d.get() + m, sizeof(double) * (size_t)m, cudaMemcpyDeviceToHost);
+    d.reset();
     if (e != cudaSuccess) {
       cudaGetLastError();
       return e == cudaErrorMemoryAllocation ? fail(ICIKT_ERR_ALLOC, "device allocation for p.adjust failed")
