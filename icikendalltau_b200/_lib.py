@@ -19,6 +19,7 @@ ERR_NO_DEVICE, ERR_BAD_ARG, ERR_TOO_LONG, ERR_CUDA, ERR_ALLOC, ERR_LIMIT = -1, -
 NCOUNTS = 7
 TOPK_BY = {"abs": 0, "signed": 1}
 TOPK_MAX = 1024
+COUNT_FILTERS_MAX = 64
 KERNEL_TILED, KERNEL_NAIVE = 0, 1
 PERSPECTIVE = {"global": 0, "local": 1, "complete": 2}
 ALTERNATIVE = {"two.sided": 0, "less": 1, "greater": 2}
@@ -46,6 +47,8 @@ EXPORTS = [
     "icikt_cross_pairs_multi", "icikt_cross_edges_multi", "icikt_cross_topk_multi",
     "icikt_p_adjust", "icikt_all_pairs_edges_padj", "icikt_all_pairs_edges_padj_multi", "icikt_cross_edges_padj",
     "icikt_cross_edges_padj_multi", "icikt_edges_copy_padj", "icikt_edges_n_tests",
+    "icikt_all_pairs_count_edges", "icikt_all_pairs_count_edges_multi", "icikt_cross_count_edges",
+    "icikt_cross_count_edges_multi",
 ]
 NSTATUS = 10
 
@@ -228,6 +231,14 @@ def load():
     for name, lead in (("icikt_all_pairs_edges_padj", one), ("icikt_cross_edges_padj", cross)):
         getattr(L, name).argtypes = lead + ef
         getattr(L, name + "_multi").argtypes = lead + [_ip, ctypes.c_int32] + ef
+        getattr(L, name).restype = getattr(L, name + "_multi").restype = ctypes.c_int
+    # the edge-count calls: (filters, n_filters, n_pass, degree or x_degree + y_degree, status_counts, max_taumax,
+    # timings) after opts, or after (devices, n_devices) for the _multi twins
+    cnt = [ctypes.POINTER(EdgeFilter), ctypes.c_int32, _lp]
+    tail = [_lp, _dp, ctypes.POINTER(Timings)]
+    for name, lead, deg in (("icikt_all_pairs_count_edges", one, [_lp]), ("icikt_cross_count_edges", cross, [_lp, _lp])):
+        getattr(L, name).argtypes = lead + cnt + deg + tail
+        getattr(L, name + "_multi").argtypes = lead + [_ip, ctypes.c_int32] + cnt + deg + tail
         getattr(L, name).restype = getattr(L, name + "_multi").restype = ctypes.c_int
     L.icikt_p_adjust.argtypes = [_dp, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, _dp, ctypes.POINTER(ctypes.c_int64)]
     L.icikt_p_adjust.restype = ctypes.c_int
@@ -616,6 +627,66 @@ def run_cross_edges(x, y, global_na=(), min_abs_cor=None, max_pvalue=None, scale
     out = _edges_out(L, h, adj is not None)
     out.update(max_taumax=mx.value, timings=t.as_dict())
     return out
+
+
+def _count_filters(filters):
+    """the icikt_edge_filter array of an edge-count call from a sequence of (min_abs_cor, max_pvalue), None as no
+    bound; an empty or too long list reaches the library as it is and is refused there"""
+    fl = [(None, None) if f is None else tuple(f) for f in filters]
+    if any(len(f) != 2 for f in fl):
+        raise ValueError("every filter is a pair (min_abs_cor, max_pvalue), None as no bound")
+    arr = (EdgeFilter * max(len(fl), 1))()
+    for k, (t, a) in enumerate(fl):
+        arr[k] = EdgeFilter(_bound(t), _bound(a), 0, 0, 0)
+    return arr, len(fl)
+
+
+def run_count_edges(data, global_na=(), filters=((None, None),), devices=None, want_degree=True, **opt_kw):
+    """icikt_all_pairs_count_edges: for every filter (min_abs_cor, max_pvalue) of `filters` (None: no bound), the
+    number of pairs that pass it -- exactly the rows run_edges(..., scale_max=False) returns with that filter -- and
+    every column's degree among them, in one walk of the pair order; no pair comes back.  data may be a scipy.sparse
+    matrix.  devices: list of CUDA ordinals -> icikt_all_pairs_count_edges_multi, bit for bit the single-device
+    result.  Returns a dict with n_pass (T,) int64, degree (C, T) int64 (a diagonal pair counts once; None without
+    want_degree), status_counts (NSTATUS,) int64 (pairs per status class), max_taumax and timings."""
+    L = load()
+    arr, T = _count_filters(filters)
+    xi, n, C, keep_alive = _input(data)
+    msfx, dargs, dev = _devices_args(devices)
+    o = make_opts(**opt_kw)
+    n_pass = np.zeros(max(T, 1), dtype=np.int64)
+    degree = np.zeros((C, max(T, 1)), dtype=np.int64) if want_degree else None
+    hist = np.zeros(NSTATUS, dtype=np.int64)
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(getattr(L, "icikt_all_pairs_count_edges" + msfx)(ctypes.byref(xi), n, gp, ng, ctypes.byref(o), *dargs, arr,
+                                                           T, _ptr(n_pass), _ptr(degree), _ptr(hist), ctypes.byref(mx),
+                                                           ctypes.byref(t)))
+    return dict(n_pass=n_pass, degree=degree, status_counts=hist, max_taumax=mx.value, timings=t.as_dict())
+
+
+def run_cross_count_edges(x, y, global_na=(), filters=((None, None),), devices=None, want_degree=True, **opt_kw):
+    """icikt_cross_count_edges: run_count_edges over the cross order of x against y (the rows run_cross_edges(...,
+    scale_max=False) returns).  devices -> icikt_cross_count_edges_multi, bit for bit the single-device result.
+    Returns a dict with n_pass (T,), x_degree (Cx, T), y_degree (Cy, T) (None without want_degree), status_counts,
+    max_taumax and timings."""
+    L = load()
+    arr, T = _count_filters(filters)
+    xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
+    msfx, dargs, dev = _devices_args(devices)
+    o = make_opts(**opt_kw)
+    n_pass = np.zeros(max(T, 1), dtype=np.int64)
+    xd = np.zeros((cx, max(T, 1)), dtype=np.int64) if want_degree else None
+    yd = np.zeros((cy, max(T, 1)), dtype=np.int64) if want_degree else None
+    hist = np.zeros(NSTATUS, dtype=np.int64)
+    mx = ctypes.c_double(float("nan"))
+    t = Timings()
+    g, gp, ng = _global_na_array(global_na)
+    check(getattr(L, "icikt_cross_count_edges" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
+                                                       *dargs, arr, T, _ptr(n_pass), _ptr(xd), _ptr(yd), _ptr(hist),
+                                                       ctypes.byref(mx), ctypes.byref(t)))
+    return dict(n_pass=n_pass, x_degree=xd, y_degree=yd, status_counts=hist, max_taumax=mx.value,
+                timings=t.as_dict())
 
 
 CROSS_SIDES = {"x": (True, False), "y": (False, True), "both": (True, True)}

@@ -562,6 +562,114 @@ def ici_kendalltau_cross_topk(x, y, k, by="abs", side="x", global_na=(np.nan, np
     return out
 
 
+def _bound_axis(v, arg):
+    """(the bounds of one argument of the edge-count functions, whether it spans an axis of the grid): a scalar or
+    None is one bound and no axis, a 1-D sequence one axis of its bounds"""
+    def one(b):
+        if b is None:
+            return None
+        if isinstance(b, (bool, np.bool_)) or not isinstance(b, (int, float, np.integer, np.floating)):
+            raise TypeError(f"`{arg}` takes numbers or None, got {b!r}")
+        if np.isnan(b):
+            raise ValueError(f"`{arg}` must not be NaN: None is no bound")
+        return float(b)
+    if v is None or np.ndim(v) == 0 and not isinstance(v, (str, bytes)):
+        return [one(v)], False
+    if isinstance(v, (str, bytes)) or np.ndim(v) != 1:
+        raise TypeError(f"`{arg}` takes a number, None or a 1-D sequence of them, got {v!r}")
+    vals = [one(b) for b in v]
+    if not vals:
+        raise ValueError(f"`{arg}` is an empty sequence")
+    return vals, True
+
+
+def _count_grid(min_abs_cor, max_pvalue):
+    """(the filters of the grid of min_abs_cor x max_pvalue in C order, the grid's shape)"""
+    ts, t_axis = _bound_axis(min_abs_cor, "min_abs_cor")
+    ps, p_axis = _bound_axis(max_pvalue, "max_pvalue")
+    if len(ts) * len(ps) > _lib.COUNT_FILTERS_MAX:
+        raise ValueError(f"the grid of `min_abs_cor` x `max_pvalue` has {len(ts) * len(ps)} filters; at most "
+                         f"{_lib.COUNT_FILTERS_MAX} are counted in one call")
+    shape = tuple(len(v) for v, axis in ((ts, t_axis), (ps, p_axis)) if axis)
+    return [(t, p) for t in ts for p in ps], shape
+
+
+def ici_kendalltau_edge_counts(data_matrix, min_abs_cor=None, max_pvalue=None, global_na=(np.nan, np.inf, 0),
+                               perspective="global", diag_good=True, alternative="two.sided", continuity=False,
+                               colnames=None, device=0, n_gpus=1):
+    """How many rows ici_kendalltau(..., return_matrix=False, scale_max=False, min_abs_cor=t, max_pvalue=p) would
+    return, and each sample's degree among them, for a whole grid of thresholds in one pass over the pairs -- the
+    counts a network threshold is chosen from, without the rows.
+
+    min_abs_cor and max_pvalue each take a number, None (no bound) or a 1-D sequence; the sequences span the grid
+    (their outer product, at most 64 filters, min_abs_cor first).  The pairs are counted on the device window by
+    window (_lib.run_count_edges), so neither memory nor the result grows with the number of pairs.  The rows the
+    counts stand for are those of the filtered long table with scale_max=False: the pairs that pass (degenerate pairs
+    never do) and, with diag_good=True, the diagonal rows appended on the host (p = 0, cor = n_good / max(n_good)),
+    filtered on the host with the same bounds.  A scaled threshold t is the raw threshold t * max_taumax.  Each
+    degenerate class of pairs warns once.  n_gpus > 1 spreads the pairs over GPUs 0..n_gpus-1 in one library call,
+    with the same counts as one GPU.
+
+    Returns a dict with `n_edges` (int64, the grid's shape: () for two scalars), `degree` (C x the grid's shape:
+    the rows that have the sample as s1 or s2, a diagonal row counting once), `names`, `min_abs_cor`, `max_pvalue`
+    (the grid's bounds), `max_taumax` and `run_time`.
+    """
+    filters, shape = _count_grid(min_abs_cor, max_pvalue)
+    data, names = _colnames_of(data_matrix, colnames, "data_matrix")
+    n, C = data.shape
+    if C < 2 and diag_good:
+        raise ValueError("No comparisons to do. Check the list of column names in `include_only` vs those in the "
+                         "samples.")
+    global_na = [float(v) for v in global_na]
+    kw = dict(perspective=perspective, alternative=alternative, continuity=continuity, device=device)
+    if n_gpus > 1:
+        kw["devices"] = range(n_gpus)
+    log.info("Counting edges ...")
+    t1 = time.perf_counter()
+    r = _lib.run_count_edges(data, global_na, filters, include_diag=not diag_good, **kw)
+    run_time = time.perf_counter() - t1
+    _warn_status_counts(r["status_counts"])
+    n_edges, degree = r["n_pass"], r["degree"]
+    if diag_good:  # R/kendalltau.R:374-386: the diagonal rows, masked as ici_kendalltau masks them
+        _, n_good = _keep_and_n_good(data, global_na)
+        dg = n_good / n_good.max()
+        dp = np.zeros(C)
+        for f, (t, p) in enumerate(filters):
+            sel = _edge_mask(dg, dp, t, p)
+            n_edges[f] += int(sel.sum())
+            degree[sel, f] += 1
+    return dict(n_edges=n_edges.reshape(shape), degree=degree.reshape((C,) + shape), names=names,
+                min_abs_cor=min_abs_cor, max_pvalue=max_pvalue, max_taumax=r["max_taumax"], run_time=run_time)
+
+
+def ici_kendalltau_cross_edge_counts(x, y, min_abs_cor=None, max_pvalue=None, global_na=(np.nan, np.inf, 0),
+                                     perspective="global", alternative="two.sided", continuity=False, xnames=None,
+                                     ynames=None, device=0, n_gpus=1):
+    """ici_kendalltau_edge_counts for the pairs of x's samples with y's: how many rows
+    ici_kendalltau_cross(x, y, return_matrix=False, scale_max=False, min_abs_cor=t, max_pvalue=p) would return, for
+    the grid of min_abs_cor x max_pvalue, counted on the device (_lib.run_cross_count_edges).  n_gpus > 1 spreads
+    the pairs over that many GPUs, with the same counts as one.
+
+    Returns a dict with `n_edges` (the grid's shape), `x_degree` (Cx x the grid's shape: rows with x's sample as
+    s1), `y_degree` (Cy x the grid's shape: rows with y's sample as s2), `xnames`, `ynames`, `min_abs_cor`,
+    `max_pvalue`, `max_taumax` and `run_time`.
+    """
+    filters, shape = _count_grid(min_abs_cor, max_pvalue)
+    x, y, xnames, ynames = _cross_data(x, y, xnames, ynames)
+    global_na = [float(v) for v in global_na]
+    kw = dict(perspective=perspective, alternative=alternative, continuity=continuity, device=device)
+    if n_gpus > 1:
+        kw["devices"] = range(n_gpus)
+    log.info("Counting edges ...")
+    t1 = time.perf_counter()
+    r = _lib.run_cross_count_edges(x, y, global_na, filters, **kw)
+    run_time = time.perf_counter() - t1
+    _warn_status_counts(r["status_counts"])
+    return dict(n_edges=r["n_pass"].reshape(shape), x_degree=r["x_degree"].reshape((x.shape[1],) + shape),
+                y_degree=r["y_degree"].reshape((y.shape[1],) + shape), xnames=xnames, ynames=ynames,
+                min_abs_cor=min_abs_cor, max_pvalue=max_pvalue, max_taumax=r["max_taumax"], run_time=run_time)
+
+
 _NA_METHODS = ("all.obs", "complete.obs", "pairwise.complete.obs", "everything", "na.or.complete")
 
 

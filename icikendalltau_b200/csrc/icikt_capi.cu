@@ -294,6 +294,9 @@ struct icikt_plan {
   DeviceArray<int32_t> d_mn;     // [C] entries kept per column of the block
   DeviceArray<int32_t> d_midx;   // [entries]
   DeviceArray<double> d_mlist;   // 4 x [entries]: raw, pvalue, taumax, completeness
+  // Edge-count calls (icikt_all_pairs_count_edges), summed over the windows: [16] pairs per status class, [T] passing
+  // pairs per filter, then, if degrees are wanted, [T][C] degrees (filter-major)
+  DeviceArray<unsigned long long> d_ecount;
 
   Event ev[9];
   icikt_timings tm{};
@@ -2037,6 +2040,66 @@ static void topk_sides_finish(std::vector<TopkSide>& sides, int k, Held&& held, 
   }
 }
 
+// ---- edge counts (icikt_all_pairs_count_edges, icikt_cross_count_edges): per window, the tally kernel adds the
+// window's passing pairs to the plan's counters; nothing comes back until the last window.
+static_assert(kCountFiltersMax == ICIKT_COUNT_FILTERS_MAX, "the tally kernel takes every filter in its parameters");
+struct CountSpec {
+  int T = 0;
+  double t[kCountFiltersMax], a[kCountFiltersMax];  // min_abs_cor, max_pvalue of every filter (NaN: no condition)
+  bool degree = false;                              // the caller wants degrees
+};
+
+// one of the caller's degree tables: plan columns [c_lo, c_hi), entry (c - c_lo) * T + f (may be null)
+struct DegreeOut {
+  int64_t* out;
+  int64_t c_lo, c_hi;
+};
+
+// The edge-count walk over pairs [first, last) of `order`: the counters start at zero and every window's tally adds
+// to them; then they come back once into `out` (d_ecount's layout) and d2h_ms receives the time of that copy.
+template <class Order>
+static int count_walk(icikt_plan* p, const Order& order, const CountSpec& cs, int64_t first, int64_t last, int64_t W,
+                      WalkTotals& tot, std::vector<unsigned long long>& out, float& d2h_ms) {
+  const size_t entries = 16 + (size_t)cs.T + (cs.degree ? (size_t)cs.T * (size_t)p->C : 0);
+  ECK(p->d_ecount.reserve(entries));
+  unsigned long long* c = p->d_ecount.get();
+  CK(cudaMemsetAsync(c, 0, sizeof(unsigned long long) * entries, p->stream));
+  auto select = [&](int64_t, int, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
+    EdgeTally et;
+    et.units = units;
+    et.n_units = n_units;
+    et.n_slots = n_slots;
+    et.tau = p->d_tau;
+    et.pvalue = p->d_p;
+    et.status = p->d_status;
+    et.n_filters = cs.T;
+    et.C = p->C;
+    std::memcpy(et.min_abs_cor, cs.t, sizeof(et.min_abs_cor));
+    std::memcpy(et.max_pvalue, cs.a, sizeof(et.max_pvalue));
+    et.status_counts = c;
+    et.n_pass = c + 16;
+    et.degree = cs.degree ? c + 16 + cs.T : nullptr;
+    const int l = launch_edge_tally(et, p->stream);
+    if (l < 0) return launch_fail("edge tally kernel");
+    tot.launches += l;
+    return ICIKT_OK;
+  };
+  int rc = walk_windows(p, order, first, last, W, tot, select, [](int64_t, int) { return ICIKT_OK; });
+  if (rc != ICIKT_OK) return rc;
+  try {
+    out.resize(entries);
+  } catch (const std::bad_alloc&) {
+    return fail(ICIKT_ERR_ALLOC, "out of host memory for the counters");
+  }
+  CK(cudaEventRecord(p->ev[6], p->stream));
+  rc = staged_copy_out(p, out.data(), c, sizeof(unsigned long long) * entries, p->stream);
+  if (rc != ICIKT_OK) return rc;
+  CK(cudaEventRecord(p->ev[7], p->stream));
+  CK(cudaEventSynchronize(p->ev[7]));
+  d2h_ms = ev_ms(p->ev[6], p->ev[7]);
+  return ICIKT_OK;
+}
+
 extern "C" {
 
 int64_t icikt_edges_count(const icikt_edges* e) { return e ? (int64_t)e->rows.size() : 0; }
@@ -3181,6 +3244,115 @@ int cross_edges_padj_impl(const icikt_input* x, const icikt_input* y, int64_t n,
   return edges_run(J, *filter, out, max_taumax, timings, adjust);
 }
 
+// ---- the edge-count calls: the all-pairs or cross job of the filtered calls, with counters instead of rows
+
+// the filters and n_pass of an edge-count call, checked on the host before any device is touched
+int check_count_filters(const icikt_edge_filter* filters, int32_t n_filters, const int64_t* n_pass, bool degree,
+                        CountSpec* cs) {
+  if (n_filters < 1 || n_filters > ICIKT_COUNT_FILTERS_MAX)
+    return fail(ICIKT_ERR_BAD_ARG, "n_filters must be in [1, ICIKT_COUNT_FILTERS_MAX]");
+  if (!filters) return fail(ICIKT_ERR_BAD_ARG, "filters is NULL");
+  if (!n_pass) return fail(ICIKT_ERR_BAD_ARG, "n_pass is NULL");
+  for (int32_t f = 0; f < n_filters; ++f) {
+    const std::string at = "filter " + std::to_string(f) + ": ";
+    if (filters[f].scale_max != 0)
+      return fail(ICIKT_ERR_BAD_ARG, at + "scaled thresholds are not counted (scale_max must be 0): count the raw "
+                                          "threshold t * max_taumax instead");
+    if (filters[f].max_edges != 0) return fail(ICIKT_ERR_BAD_ARG, at + "max_edges must be 0: a count returns no rows");
+    if (filters[f].reserved != 0) return fail(ICIKT_ERR_BAD_ARG, at + "reserved must be 0");
+    cs->t[f] = filters[f].min_abs_cor;
+    cs->a[f] = filters[f].max_pvalue;
+  }
+  cs->T = n_filters;
+  cs->degree = degree;
+  return ICIKT_OK;
+}
+
+// The counting job over the devices of J, its arguments checked: every worker walks its slice with its own counters,
+// and the host sums them into the caller's arrays (integers: the sum is that of one device).  deg: the caller's
+// degree tables, each over plan columns [c_lo, c_hi).
+int count_run(MultiJob& J, const CountSpec& cs, int64_t* n_pass, const std::vector<DegreeOut>& deg,
+              int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  int rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  std::vector<std::vector<unsigned long long>> got((size_t)J.n_devices);
+  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
+  if (J.ptot > 0) {
+    std::vector<MultiWork> work;
+    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+    multi_probe_peers(J);
+    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
+      icikt_plan* p = nullptr;
+      int r = window_multi_worker(J, k, &p);
+      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
+      if (r != ICIKT_OK || hi <= lo) return r;
+      WalkTotals tot;
+      float d2h_ms = 0.f;
+      r = ensure_walk_buffers(p);
+      if (r == ICIKT_OK)
+        r = with_order(J, p, [&](const auto& order) {
+          return count_walk(p, order, cs, lo, hi, p->P, tot, got[(size_t)k], d2h_ms);
+        });
+      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
+      bits[(size_t)k] = tot.bits;
+      return r;
+    });
+    if (rc != ICIKT_OK) return rc;
+  } else {
+    no_pairs(max_taumax, timings);  // one column, no diagonal: every count is 0
+  }
+  const int T = cs.T;
+  const int64_t C = J.C;
+  auto sum = [&](size_t at) {
+    unsigned long long s = 0;
+    for (const auto& g : got)
+      if (!g.empty()) s += g[at];
+    return (int64_t)s;
+  };
+  for (int f = 0; f < T; ++f) n_pass[f] = sum(16 + (size_t)f);
+  if (status_counts)
+    for (int c = 0; c < ICIKT_NSTATUS; ++c) status_counts[c] = sum((size_t)c);
+  for (const DegreeOut& d : deg)
+    if (d.out)
+      for (int64_t c = d.c_lo; c < d.c_hi; ++c)
+        for (int f = 0; f < T; ++f) d.out[(c - d.c_lo) * T + f] = sum(16 + (size_t)T + (size_t)f * (size_t)C + (size_t)c);
+  if (J.ptot > 0 && max_taumax) *max_taumax = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  return ICIKT_OK;
+}
+
+int count_edges_impl(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na, const icikt_opts& o,
+                     const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filters, int32_t n_filters,
+                     int64_t* n_pass, int64_t* degree, int64_t* status_counts, double* max_taumax,
+                     icikt_timings* timings) {
+  ColumnSource s;
+  CountSpec cs;
+  int rc = check_count_filters(filters, n_filters, n_pass, degree != nullptr, &cs);
+  if (rc == ICIKT_OK) rc = n < 1 ? fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1") : cross_source(x, "x", n, &s);
+  if (rc == ICIKT_OK) rc = check_window_args(s, n, s.C, global_na, n_global_na, o);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  MultiJob J(n_devices);
+  J.src = s; J.n = n; J.C = s.C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.ptot = tri_pairs(s.C) + (o.include_diag ? s.C : 0);
+  return count_run(J, cs, n_pass, {DegreeOut{degree, 0, s.C}}, status_counts, max_taumax, timings);
+}
+
+int cross_count_edges_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices,
+                           const icikt_edge_filter* filters, int32_t n_filters, int64_t* n_pass, int64_t* x_degree,
+                           int64_t* y_degree, int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  ColumnSource sx, sy;
+  CountSpec cs;
+  int rc = check_count_filters(filters, n_filters, n_pass, x_degree || y_degree, &cs);
+  if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
+  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc != ICIKT_OK) return rc;
+  MultiJob J(n_devices);
+  cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
+  return count_run(J, cs, n_pass, {DegreeOut{x_degree, 0, sx.C}, DegreeOut{y_degree, sx.C, sx.C + sy.C}},
+                   status_counts, max_taumax, timings);
+}
+
 }  // namespace
 
 extern "C" {
@@ -3517,6 +3689,42 @@ int icikt_edges_copy_padj(const icikt_edges* e, double* padj) {
 }
 
 int64_t icikt_edges_n_tests(const icikt_edges* e) { return e ? e->n_tests : -1; }
+
+int icikt_all_pairs_count_edges(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                const icikt_opts* opts, const icikt_edge_filter* filters, int32_t n_filters,
+                                int64_t* n_pass, int64_t* degree, int64_t* status_counts, double* max_taumax,
+                                icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return count_edges_impl(x, n, global_na, n_global_na, o, &o.device, 1, filters, n_filters, n_pass, degree,
+                          status_counts, max_taumax, timings);
+}
+
+int icikt_all_pairs_count_edges_multi(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                      const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                      const icikt_edge_filter* filters, int32_t n_filters, int64_t* n_pass,
+                                      int64_t* degree, int64_t* status_counts, double* max_taumax,
+                                      icikt_timings* timings) {
+  return count_edges_impl(x, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filters, n_filters,
+                          n_pass, degree, status_counts, max_taumax, timings);
+}
+
+int icikt_cross_count_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filters,
+                            int32_t n_filters, int64_t* n_pass, int64_t* x_degree, int64_t* y_degree,
+                            int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return cross_count_edges_impl(x, y, n, global_na, n_global_na, o, &o.device, 1, filters, n_filters, n_pass, x_degree,
+                                y_degree, status_counts, max_taumax, timings);
+}
+
+int icikt_cross_count_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                                  int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
+                                  int32_t n_devices, const icikt_edge_filter* filters, int32_t n_filters,
+                                  int64_t* n_pass, int64_t* x_degree, int64_t* y_degree, int64_t* status_counts,
+                                  double* max_taumax, icikt_timings* timings) {
+  return cross_count_edges_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filters,
+                                n_filters, n_pass, x_degree, y_degree, status_counts, max_taumax, timings);
+}
 
 int icikt_p_adjust(const double* p, int64_t m, int32_t method, int32_t device, double* out, int64_t* n_tests) {
   if (m < 0) return fail(ICIKT_ERR_BAD_ARG, "m must be >= 0");

@@ -259,6 +259,26 @@ struct TopkDeviceMerge {
 };
 int launch_topk_device_merge(const TopkDeviceMerge& m, cudaStream_t stream);
 
+// The counting pass of the edge-count calls (icikt_select.cu), per window: every slot of the window is tested once
+// against the T filters (edge_keep_window without scale_max; NaN bounds are no condition), which travel in the launch
+// parameters; the counters add up over the windows and nothing else is written.  Degrees are filter-major and indexed
+// by the plan's column: entry f * C + c (a cross call's Y column j is the plan's column Cx + j).
+constexpr int kCountFiltersMax = 64;  // ICIKT_COUNT_FILTERS_MAX
+struct EdgeTally {
+  const PairUnit* units;  // device, the window's units (slots relative to the window)
+  int64_t n_units;
+  int64_t n_slots;        // pairs in the window
+  const double *tau, *pvalue;
+  const int32_t* status;
+  int n_filters;          // T, 1 .. kCountFiltersMax
+  int64_t C;              // columns of the plan
+  double min_abs_cor[kCountFiltersMax], max_pvalue[kCountFiltersMax];
+  unsigned long long* status_counts;  // device [16]: pairs per status class
+  unsigned long long* n_pass;         // device [T]
+  unsigned long long* degree;         // device [T C], or null
+};
+int launch_edge_tally(const EdgeTally& s, cudaStream_t stream);
+
 // R's p.adjust on the device (icikt_padj.cu, arithmetic in icikt_padj.cuh).  Each returns the first CUDA error.
 // counts[0] += the non-NaN values of p[0, n); the keys (padj_key) of those <= bound (NaN: all) are appended at
 // keys[counts[1]++], which the caller has made room for.

@@ -8,6 +8,8 @@
 //     bits below it.  Tiles without a kept slot stop after reading their 32 words.
 // HBM-bound: the count pass reads the status and, only for a bound that is given, raw (8 B) and the p-value
 // (8 B); the scatter pass reads 1/8 B of mask per slot and the fields of the kept slots.
+// The counting pass of the edge-count calls (edge_tally_kernel) tests T filters per slot in one read of the slot and
+// writes nothing but counters: per filter, the pairs that pass and every column's degree.
 // The selection of the top-k call (icikt_all_pairs_topk) follows the edge kernels: per-column buckets of the
 // candidates that beat a column's k-th entry, merged into the column's sorted list (see launch_topk_select).  Over
 // several devices, topk_device_merge_kernel folds the devices' lists of a block of columns into one.
@@ -155,6 +157,79 @@ __global__ void __launch_bounds__(kSelThreads) edge_scatter_kernel(const EdgeSel
     r.completeness = s.completeness[slot];
     s.rows[base + word_off[m] + __popc(w & ((1u << lane) - 1u))] = r;
   }
+}
+
+// The edge-count calls: one CTA per tile of kEdgeTile slots, every slot read once (status, raw, p-value) and tested
+// against all T filters into a T-bit pass mask held in registers.  Work past the mask follows the set bits only: a
+// warp whose 32 masks are all zero (few pairs pass) does no more than count its status classes.  For every filter f
+// set in some lane, one ballot gives the warp's count (summed per lane in registers, lane f % 32 owns filter f, then
+// one shared atomic per lane and one global atomic per CTA and filter); the row endpoint i is shared by the lanes of a
+// unit and usually by the whole warp, so the lanes with the same i add their count with one atomic (match_any), and
+// the other endpoint j takes one atomic per passing pair and filter.  A diagonal pair (i == j) adds 1 to its column.
+__global__ void __launch_bounds__(kSelThreads) edge_tally_kernel(const EdgeTally s) {
+  __shared__ unsigned cta_pass[kCountFiltersMax];
+  __shared__ unsigned cta_status[16];
+  __shared__ long long unit_range[2];
+  const long long tile = blockIdx.x;
+  const int lane = threadIdx.x & 31, T = s.n_filters;
+  if (threadIdx.x < kCountFiltersMax) cta_pass[threadIdx.x] = 0;
+  if (threadIdx.x < 16) cta_status[threadIdx.x] = 0;
+  if (threadIdx.x < 2) {
+    const long long first_slot = tile * kEdgeTile;
+    const long long last_slot = min((long long)s.n_slots, first_slot + kEdgeTile) - 1;
+    unit_range[threadIdx.x] = unit_of(s.units, 0, s.n_units, threadIdx.x ? last_slot : first_slot);
+  }
+  __syncthreads();
+  const long long ua = unit_range[0], ub = unit_range[1] + 1;
+  unsigned pass_lo = 0, pass_hi = 0;  // this warp's passing pairs of filters lane and lane + 32
+#pragma unroll 1
+  for (int r = 0; r < kSelRounds; ++r) {
+    const long long slot = tile * kEdgeTile + r * kSelThreads + threadIdx.x;
+    int32_t st = -1;
+    unsigned long long mask = 0;
+    if (slot < s.n_slots) {
+      st = s.status[slot];
+      if (st == 0) {
+        const double raw = s.tau[slot], pv = s.pvalue[slot];
+        for (int f = 0; f < T; ++f)
+          mask |= (unsigned long long)edge_keep_window(0, raw, pv, s.min_abs_cor[f], s.max_pvalue[f], false, 1.0) << f;
+      } else {
+        atomicAdd(&cta_status[min(st, 15)], 1u);
+      }
+    }
+    const unsigned ok = __ballot_sync(FULL, st == 0);
+    if (lane == 0 && ok) atomicAdd(&cta_status[0], (unsigned)__popc(ok));
+    const unsigned any_lo = __reduce_or_sync(FULL, (unsigned)mask), any_hi = __reduce_or_sync(FULL, (unsigned)(mask >> 32));
+    unsigned long long any = ((unsigned long long)any_hi << 32) | any_lo;
+    if (!any) continue;
+    int32_t i = -1, j = -1;
+    if (mask) {
+      const PairUnit u = s.units[unit_of(s.units, ua, ub, slot)];
+      i = u.col;
+      j = u.j0 + (int32_t)(slot - u.slot0);
+    }
+    const unsigned peers = __match_any_sync(FULL, i);
+    for (; any; any &= any - 1) {
+      const int f = __ffsll((long long)any) - 1;
+      const bool bit = (mask >> f) & 1ull;
+      const unsigned b = __ballot_sync(FULL, bit);
+      if (lane == (f & 31)) {
+        if (f < 32) pass_lo += __popc(b); else pass_hi += __popc(b);
+      }
+      if (s.degree && bit) {
+        unsigned long long* deg = s.degree + (long long)f * s.C;
+        const unsigned grp = b & peers;
+        if (lane == __ffs(grp) - 1) atomicAdd(deg + i, (unsigned long long)__popc(grp));
+        if (j != i) atomicAdd(deg + j, 1ull);
+      }
+    }
+  }
+  if (pass_lo) atomicAdd(&cta_pass[lane], pass_lo);
+  if (pass_hi) atomicAdd(&cta_pass[lane + 32], pass_hi);
+  __syncthreads();
+  if (threadIdx.x < T && cta_pass[threadIdx.x]) atomicAdd(s.n_pass + threadIdx.x, (unsigned long long)cta_pass[threadIdx.x]);
+  if (threadIdx.x < 16 && cta_status[threadIdx.x])
+    atomicAdd(s.status_counts + threadIdx.x, (unsigned long long)cta_status[threadIdx.x]);
 }
 
 // Top-k: the count pass (kScatter false) and the scatter pass (true) of one tile of kEdgeTile slots.  Both make
@@ -401,6 +476,15 @@ int launch_topk_select(const TopkSelect& s, cudaStream_t stream) {
   topk_bucket_kernel<true><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
   topk_merge_kernel<<<(unsigned)L, kMergeThreads, 0, stream>>>(s);
   return launch_status(4);
+}
+
+int launch_edge_tally(const EdgeTally& s, cudaStream_t stream) {
+  if (s.n_slots <= 0) return launch_status(0);
+  const long long tiles = (s.n_slots + kEdgeTile - 1) / kEdgeTile;
+  if (tiles > 0x7fffffffLL || s.n_filters < 1 || s.n_filters > kCountFiltersMax || s.C > 0x7fffffffLL)
+    return launch_refused("edge tally: bad arguments");
+  edge_tally_kernel<<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  return launch_status(1);
 }
 
 int launch_edge_select(const EdgeSelect& s, cudaStream_t stream) {

@@ -523,6 +523,57 @@ int icikt_edges_copy_padj(const icikt_edges* e, double* padj);
 /* m of a _padj result; -1 for NULL or a result without adjustment */
 int64_t icikt_edges_n_tests(const icikt_edges* e);
 
+/* ---- edge counts: how many pairs pass each of several edge filters, and each column's degree under each, in ONE walk
+ * of the pair order and without returning a single pair -- what a threshold would return before the filtered call is
+ * run with it (edges against threshold, degree distributions, hub and isolated columns).  The pair kernel runs once
+ * whatever the number of filters.
+ *
+ *   - Input: that of the filtered calls, all pairs of one matrix (an icikt_input, dense or CSC, whose messages name it
+ *     matrix x; the diagonal pairs follow when include_diag is set) or the cross order of X against Y.
+ *   - Filters: filters[0 .. n_filters), 1 <= n_filters <= ICIKT_COUNT_FILTERS_MAX, each an icikt_edge_filter with
+ *     scale_max = 0, reserved = 0 and max_edges = 0.  A pair passes filter f under exactly the predicate of
+ *     icikt_all_pairs_edges without scale_max: status == 0 && (isnan(min_abs_cor) || fabs(raw) >= min_abs_cor) &&
+ *     (isnan(max_pvalue) || pvalue <= max_pvalue).  Scaled thresholds are refused: whether a pair passes raw / M >= t
+ *     depends on M = max(taumax), known only after the last window, and a count has no rows to trim once it is.  The
+ *     call returns M in max_taumax, so a scaled threshold t is counted as the raw threshold t * M.  That is the
+ *     meaning of scaling here; it can differ from scale_max = 1 (fabs(raw / M) >= t) in the last ulp at the boundary.
+ *   - Outputs, caller-allocated: n_pass[T] (required) the pairs that pass each filter, icikt_edges_count of the
+ *     filtered call with that one filter; degree[C * T] (may be NULL), entry c * T + f, the passing pairs of filter f
+ *     that have column c as either endpoint, a diagonal pair (c, c) counting once; for a cross call x_degree[Cx * T]
+ *     and y_degree[Cy * T] (each may be NULL) the same over X's and Y's columns; status_counts[ICIKT_NSTATUS] (may be
+ *     NULL) the pairs per status class, as icikt_matrices returns them; max_taumax (may be NULL) M or NaN.
+ *   - Every output is an integer count independent of the order of the work, so the _multi twins ((devices, n_devices)
+ *     after opts, as the edges multi calls; per-device counts summed on the host) return bit for bit the one-device
+ *     result.
+ *   - Device memory does not depend on the number of pairs: the per-column tables, one window of pairs
+ *     (ICIKT_EDGE_WINDOW) and 8 B x (C x T + T + 16) of counters, which come back once, after the last window.
+ *   - Refused with ICIKT_ERR_BAD_ARG before any device is touched: n_filters out of range, a NULL filters or n_pass, a
+ *     filter with scale_max, max_edges or reserved != 0, and whatever the filtered call refuses of its options
+ *     (ICIKT_PERSPECTIVE_COMPLETE, ICIKT_KERNEL_NAIVE, want_counts, pair_lo / pair_hi != 0; for cross calls
+ *     include_diag), n_devices out of 1..16.
+ *   - timings (may be NULL) as in the edges calls: epilogue_ms includes the counting pass, d2h_ms is the copy of the
+ *     counters. */
+#define ICIKT_COUNT_FILTERS_MAX 64
+
+int icikt_all_pairs_count_edges(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                const icikt_opts* opts, const icikt_edge_filter* filters, int32_t n_filters,
+                                int64_t* n_pass, int64_t* degree, int64_t* status_counts, double* max_taumax,
+                                icikt_timings* timings);
+int icikt_all_pairs_count_edges_multi(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                      const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                      const icikt_edge_filter* filters, int32_t n_filters, int64_t* n_pass,
+                                      int64_t* degree, int64_t* status_counts, double* max_taumax,
+                                      icikt_timings* timings);
+int icikt_cross_count_edges(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                            int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filters,
+                            int32_t n_filters, int64_t* n_pass, int64_t* x_degree, int64_t* y_degree,
+                            int64_t* status_counts, double* max_taumax, icikt_timings* timings);
+int icikt_cross_count_edges_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                                  int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
+                                  int32_t n_devices, const icikt_edge_filter* filters, int32_t n_filters,
+                                  int64_t* n_pass, int64_t* x_degree, int64_t* y_degree, int64_t* status_counts,
+                                  double* max_taumax, icikt_timings* timings);
+
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
  * pay the copies.  A plan is bound to one device and is not thread-safe.            */
