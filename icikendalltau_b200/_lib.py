@@ -945,6 +945,13 @@ def launch_shape(n, tier=0, n_sm=148, complete_obs=False):
                 variant=("smem", "inplace", "gmem")[int(out[3])], cap=int(out[4]), stage_rows=int(out[5]))
 
 
+def pass_a_radix(n):
+    """whether pass A runs radix-16 levels at length n (host only; the same for every tier)"""
+    out = np.zeros(8, dtype=np.int32)
+    check(load().icikt_launch_shape(int(n), 0, 148, 0, out.ctypes.data))
+    return bool(out[6])
+
+
 def pair_from_index(C, index, include_diag=False):
     i, j = ctypes.c_int32(), ctypes.c_int32()
     check(load().icikt_pair_from_index(C, int(bool(include_diag)), int(index), ctypes.byref(i), ctypes.byref(j)))

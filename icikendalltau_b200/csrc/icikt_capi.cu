@@ -1478,6 +1478,7 @@ int icikt_launch_shape(int64_t n, int32_t tier, int32_t n_sm, int32_t complete_o
   out[4] = cap;
   // in place: rows of the other column's rank table one staging part holds (the counter area behind the sequence)
   out[5] = sh.inplace_kk != 0 ? (int)std::min<int64_t>((n + 63) & ~63LL, ((sh.region_bytes - 2 * cap) >> 1) & ~63) : 0;
+  out[6] = sh.radix ? 1 : 0;
   return ICIKT_OK;
 }
 

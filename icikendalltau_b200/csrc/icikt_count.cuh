@@ -199,6 +199,56 @@ struct Mem<false> {
         : "+r"(s.C), "+r"(s.D2), "+r"(s.D3a), "+r"(s.D3b), "+r"(s.acc)
         : "r"(w), "r"(a2), "r"(a3), "n"(8u << SH), "n"(2u << SH), "n"(1u << SH));
   }
+  // step16 at a bit position known at run time only (a radix-16 level, see radix_level): m8 / m2 / m1 are the
+  // masks of the key's digit bits 3 / 1 / 0 in w
+  static __device__ __forceinline__ void step16_at(NibbleCounts& s, uint32_t w, uint32_t a2, uint32_t a3, uint32_t m8,
+                                                   uint32_t m2, uint32_t m1) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p3, p1, p0;\n\t"
+        ".reg .b32 t, W1, W2, W3, Ds;\n\t"
+        "and.b32 t, %5, %8;\n\t"
+        "setp.ne.u32 p3, t, 0;\n\t"
+        "and.b32 t, %5, %9;\n\t"
+        "setp.ne.u32 p1, t, 0;\n\t"
+        "and.b32 t, %5, %10;\n\t"
+        "setp.ne.u32 p0, t, 0;\n\t"
+        "selp.b32 W1, 0x02010000, 0x01010100, p3;\n\t"
+        "dp4a.u32.u32 %4, %0, W1, %4;\n\t"
+        "shf.l.wrap.b32 W2, 0, 1, %6;\n\t"
+        "add.u32 %0, %0, W2;\n\t"
+        "dp4a.u32.u32 %4, %1, W2, %4;\n\t"
+        "@p1 add.u32 %1, %1, W2;\n\t"
+        "shf.l.wrap.b32 W3, 0, 1, %7;\n\t"
+        "selp.b32 Ds, %3, %2, p3;\n\t"
+        "dp4a.u32.u32 %4, Ds, W3, %4;\n\t"
+        "selp.b32 W3, W3, 0, p0;\n\t"
+        "@p3 add.u32 %3, %3, W3;\n\t"
+        "@!p3 add.u32 %2, %2, W3;\n\t"
+        "}"
+        : "+r"(s.C), "+r"(s.D2), "+r"(s.D3a), "+r"(s.D3b), "+r"(s.acc)
+        : "r"(w), "r"(a2), "r"(a3), "r"(m8), "r"(m2), "r"(m1));
+  }
+  // one key of a radix-16 level's scatter: its digit d = (key >> s) & 15 selects this thread's slot counter
+  // cnt[d] (u16, at me + d * row), the key goes to that slot of buffer `base` and the counter moves on.  The
+  // key's high 16 bits are ignored.  8 instructions, three of them on the FMA pipe.
+  static __device__ __forceinline__ void scatter16(uint32_t key, uint32_t s, uint32_t me, uint32_t row, ptr base,
+                                                   const PipeConst& pc) {
+    asm volatile(
+        "{\n\t"
+        ".reg .b32 d, ca, sl, ad;\n\t"
+        "shr.b32 d, %0, %1;\n\t"
+        "and.b32 d, d, 15;\n\t"
+        "mad.lo.u32 ca, d, %3, %2;\n\t"
+        "ld.shared.u16 sl, [ca];\n\t"
+        "mad.lo.u32 ad, sl, %5, %4;\n\t"
+        "st.shared.u16 [ad], %0;\n\t"
+        "mad.lo.u32 sl, %6, %6, sl;\n\t"
+        "st.shared.u16 [ca], sl;\n\t"
+        "}" ::"r"(key),
+        "r"(s), "r"(me), "r"(row), "r"(base), "r"(pc.two), "r"(pc.one)
+        : "memory");
+  }
   static __device__ __forceinline__ void red_add32(ptr p, uint32_t v) {
     asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(p), "r"(v) : "memory");
   }
@@ -328,6 +378,24 @@ __device__ __forceinline__ void nibble_word(NibbleCounts& s, uint32_t w) {
   Mem<G>::template step16<16>(s, w, a2 >> 16, a3 >> 16);
 }
 
+// this thread's share of a nibble-tree count (see nibble_level) from its sweep's counts s, the ones r at the
+// root and the ones E[] before its range, packed as nibble_level's q[]
+__device__ __forceinline__ uint32_t nibble_share(const NibbleCounts& s, const uint32_t R, const uint32_t r,
+                                                 const uint32_t E[8]) {
+  // zeros per node: b1 = 0 per (b3 b2), then b0 = 0 per (b3 b2 b1) (bytewise, no borrows)
+  const uint32_t N2 = s.C - s.D2;
+  const uint32_t N3a = __byte_perm(N2, s.D2, 0x5140) - s.D3a, N3b = __byte_perm(N2, s.D2, 0x7362) - s.D3b;
+  uint32_t x = (R - r) * E[1];
+  x = __dp2a_lo(E[0], __byte_perm(s.C, 0u, 0x4420), x);  // c0 * E(c1) + c2 * E(c3)
+  x = __dp2a_hi(E[3], N2, __dp2a_lo(E[2], N2, x));
+  x = __dp2a_hi(E[5], N3a, __dp2a_lo(E[4], N3a, x));
+  x = __dp2a_hi(E[7], N3b, __dp2a_lo(E[6], N3b, x));
+  // sum of C(n1, 2) = (sum n1^2 - sum n1) / 2 over the 15 nodes
+  const uint32_t sq = __dp4a(s.D2, s.D2, __dp4a(s.D3a, s.D3a, __dp4a(s.D3b, s.D3b, __dp4a(s.C & 0xff00ff00u, s.C, r * r))));
+  const uint32_t li = __dp4a(s.D2, 0x01010101u, __dp4a(s.D3a, 0x01010101u, __dp4a(s.D3b, 0x01010101u, __dp4a(s.C, 0x01000100u, r))));
+  return s.acc + x - ((sq - li) >> 1);
+}
+
 // The low-nibble level after its sweep: this thread's share is
 //   acc - sum over nodes of C(n1, 2)                    (within the range)
 //   + sum over nodes of n0 * (ones at the node in earlier ranges)
@@ -371,21 +439,125 @@ __device__ __forceinline__ void nibble_level(const NibbleCounts& s, const uint32
   uint32_t E[8];  // ones before the range (exclusive prefix over the CTA; below 65 536)
 #pragma unroll
   for (int k = 0; k < 8; ++k) E[k] = __reduce_add_sync(FULL, v[k]) + incl[k] - q[k];
-  if (!idle) {
-    // zeros per node: b1 = 0 per (b3 b2), then b0 = 0 per (b3 b2 b1) (bytewise, no borrows)
-    const uint32_t N2 = s.C - s.D2;
-    const uint32_t N3a = __byte_perm(N2, s.D2, 0x5140) - s.D3a, N3b = __byte_perm(N2, s.D2, 0x7362) - s.D3b;
-    uint32_t x = (R - r) * E[1];
-    x = __dp2a_lo(E[0], __byte_perm(s.C, 0u, 0x4420), x);  // c0 * E(c1) + c2 * E(c3)
-    x = __dp2a_hi(E[3], N2, __dp2a_lo(E[2], N2, x));
-    x = __dp2a_hi(E[5], N3a, __dp2a_lo(E[4], N3a, x));
-    x = __dp2a_hi(E[7], N3b, __dp2a_lo(E[6], N3b, x));
-    // sum of C(n1, 2) = (sum n1^2 - sum n1) / 2 over the 15 nodes
-    const uint32_t sq = __dp4a(s.D2, s.D2, __dp4a(s.D3a, s.D3a, __dp4a(s.D3b, s.D3b, __dp4a(s.C & 0xff00ff00u, s.C, r * r))));
-    const uint32_t li = __dp4a(s.D2, 0x01010101u, __dp4a(s.D3a, 0x01010101u, __dp4a(s.D3b, 0x01010101u, __dp4a(s.C, 0x01000100u, r))));
-    acc64 += (unsigned long long)(s.acc + x - ((sq - li) >> 1));
-  }
+  if (!idle) acc64 += (unsigned long long)nibble_share(s, R, r, E);
   __syncthreads();  // the warp totals are read before anybody reuses the buffer
+}
+
+// The 16 digit counts (b3 b2 b1 b0) of N keys whose node ones counts are e[] (packed as nibble_level's q[]):
+// each node splits its keys into the ones and the rest, from the root down.
+__device__ __forceinline__ void nibble_digits(uint32_t N, const uint32_t e[8], uint32_t dig[16]) {
+  const uint32_t c1 = e[0] & 0xffffu, c3 = e[0] >> 16, r = e[1];
+  const uint32_t cls[4] = {N - r - c1, c1, r - c3, c3};
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    const uint32_t d2 = (e[2 + (c >> 1)] >> (16 * (c & 1))) & 0xffffu;
+    const uint32_t pre[2] = {cls[c] - d2, d2};
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int p = 2 * c + h;
+      const uint32_t d3 = (e[4 + (p >> 1)] >> (16 * (p & 1))) & 0xffffu;
+      dig[2 * p] = pre[h] - d3;
+      dig[2 * p + 1] = d3;
+    }
+  }
+}
+
+// A radix-16 level of pass A on bits s+3 .. s (s >= 4, shared memory only): the count of the nibble level at
+// bit s -- the same tree over the same order, so it counts what the two two-bit levels it replaces count on
+// those bits, up to terms of column y alone -- and a stable partition of the sequence by the 4-bit digit.
+//   sweep 1  the nibble tree over the range (step16_at);
+//   one warp scan of the 15 node ones counts, the warps' totals through `tot` (32 bytes per warp), gives the
+//            count's cross-range share and, split node by node (nibble_digits), every digit's keys before the
+//            range and in the whole buffer; the start slot of each digit goes to this thread's column of the
+//            u16 counter table cnt[16][T] at `ctr` (odd threads' counters 64 bytes further on, so that a warp's
+//            even lanes hit banks 0-15 and its odd lanes banks 16-31 whatever their digits: conflict-free; the
+//            last row's odd counters run 64 bytes past the table);
+//   sweep 2  stores every key to slot cnt[d][tid]++ of the other buffer (scatter16).
+// Threads outside the sequence (TAIL) enter the scan with the counts of R padding keys, digit 15.  Two
+// block-wide barriers.
+template <bool TAIL>
+__device__ __forceinline__ void radix_level(const uint32_t a, const uint32_t b, const uint32_t ctr, const uint32_t s,
+                                            const int kk, const int nwarps, const bool idle, const bool tail,
+                                            const int lane, const int warp, const PipeConst& pc,
+                                            unsigned long long& acc64) {
+  typedef Mem<false> M;
+  const uint32_t T = (uint32_t)nwarps << 5, tid = ((uint32_t)warp << 5) + (uint32_t)lane;
+  const uint32_t R = (uint32_t)kk << 3, my_pos = tid * R, ra = a + tid * (R << 1);
+  const uint32_t tot = ctr + (T << 5) + 64u;
+  NibbleCounts nc = {0u, 0u, 0u, 0u, 0u};
+  if (TAIL && tail) nc.C = nc.D2 = nc.D3b = R << 24;
+  {
+    uint32_t m8 = 8u << s, m2 = 2u << s, m1 = 1u << s;
+    uint32_t h8 = m8 << 16, h2 = m2 << 16, h1 = m1 << 16;
+    const uint32_t s2 = s - 1u, s3 = s - 2u;
+#pragma unroll 1
+    for (int c = 0; c < (idle ? 0 : kk); ++c) {
+      uint32_t w[4];
+      M::ld128(ra + (c << 4), w[0], w[1], w[2], w[3]);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const uint32_t a2 = (w[j] >> s2) & 0x00180018u, a3 = (w[j] >> s3) & 0x00180018u;
+        M::step16_at(nc, w[j], a2, a3, m8, m2, m1);
+        M::step16_at(nc, w[j], a2 >> 16, a3 >> 16, h8, h2, h1);
+      }
+    }
+  }
+  const uint32_t r = ((nc.C >> 16) & 0xffu) + (nc.C >> 24);
+  const uint32_t q[8] = {__byte_perm(nc.C, 0u, 0x4341),   r,
+                         __byte_perm(nc.D2, 0u, 0x4140),  __byte_perm(nc.D2, 0u, 0x4342),
+                         __byte_perm(nc.D3a, 0u, 0x4140), __byte_perm(nc.D3a, 0u, 0x4342),
+                         __byte_perm(nc.D3b, 0u, 0x4140), __byte_perm(nc.D3b, 0u, 0x4342)};
+  uint32_t incl[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) incl[k] = q[k];
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      const uint32_t t = __shfl_up_sync(FULL, incl[k], d);
+      if (lane >= d) incl[k] += t;
+    }
+  }
+  if (lane == 31) {
+    M::st128(tot + ((uint32_t)warp << 5), incl[0], incl[1], incl[2], incl[3]);
+    M::st128(tot + ((uint32_t)warp << 5) + 16u, incl[4], incl[5], incl[6], incl[7]);
+  }
+  __syncthreads();
+  uint32_t v[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
+  if (lane < nwarps) {
+    M::ld128(tot + ((uint32_t)lane << 5), v[0], v[1], v[2], v[3]);
+    M::ld128(tot + ((uint32_t)lane << 5) + 16u, v[4], v[5], v[6], v[7]);
+  }
+  uint32_t E[8], N[8];  // ones before the range / in the whole buffer, per node
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    E[k] = __reduce_add_sync(FULL, (lane < warp) ? v[k] : 0u) + incl[k] - q[k];
+    N[k] = __reduce_add_sync(FULL, v[k]);
+  }
+  if (!idle) {
+    acc64 += (unsigned long long)nibble_share(nc, R, r, E);
+    uint32_t before[16], total[16];
+    nibble_digits(my_pos, E, before);
+    nibble_digits(T * R, N, total);
+    const uint32_t me = ctr + (tid << 1) + ((tid & 1u) << 6), row = T << 1;
+    uint32_t run = 0u;
+#pragma unroll
+    for (int d = 0; d < 16; ++d) {
+      M::st16(me + (uint32_t)d * row, run + before[d]);
+      run += total[d];
+    }
+#pragma unroll 1
+    for (int c = 0; c < kk; ++c) {
+      uint32_t w[4];
+      M::ld128(ra + (c << 4), w[0], w[1], w[2], w[3]);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        M::scatter16(w[j], s, me, row, b, pc);
+        M::scatter16(M::hi16(w[j], pc.c64k), s, me, row, b, pc);
+      }
+    }
+  }
+  __syncthreads();  // the next level reads the other buffer; also protects `tot`
 }
 
 // block-wide barriers count_pass executes for L bits (threads that skip it must keep them)
@@ -408,8 +580,11 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
                                            const int nwarps, const int L, uint32_t* descA, uint32_t* descB,
                                            const int lane, const int warp, const PipeConst pc,
                                            unsigned long long& acc64, const uint32_t lead = 0u,
-                                           const uint32_t len = 0u) {
+                                           const uint32_t len = 0u, const uint32_t ctr = 0u) {
   typedef Mem<G> M;
+  // ctr != 0 (shared memory only): the bits from 4 up to the highest multiple of 4 below L take radix-16
+  // levels (radix_level, counter table at ctr), the two-bit levels only the bits above them
+  const int nr = (!G && ctr != 0u && L > 4) ? (L - 4) >> 2 : 0;
   const uint32_t tid = ((uint32_t)warp << 5) + (uint32_t)lane;
   const uint32_t R = (uint32_t)kk << 3;                // keys per thread range
   const uint32_t my_off = tid * (R << 1);              // bytes
@@ -426,7 +601,7 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     const typename M::ptr rb = M::add(b, (int32_t)my_off);
     for (int c = 0; c < kk; ++c) M::st128(M::add(rb, c << 4), 0u, 0u, 0u, 0u);
   }
-  for (int s = (L - 1) & ~1; s >= 4; s -= 2) {
+  for (int s = (L - 1) & ~1; s >= 4 + 4 * nr; s -= 2) {
     const typename M::ptr ra = M::add(a, (int32_t)my_off);
     uint32_t cl = 0, cb = 0, wm = 0, m4 = 0;
     uint32_t chj[4] = {0u, 0u, 0u, 0u};
@@ -503,6 +678,14 @@ __device__ __forceinline__ void count_pass(typename Mem<G>::ptr a, typename Mem<
     const typename M::ptr t = a;
     a = b;
     b = t;
+  }
+  if constexpr (!G) {
+    for (int s = 4 * nr; s >= 4; s -= 4) {
+      radix_level<TAIL>(a, b, ctr, (uint32_t)s, kk, nwarps, idle, tail, lane, warp, pc, acc64);
+      const uint32_t t = a;
+      a = b;
+      b = t;
+    }
   }
   NibbleCounts nc = {0u, 0u, 0u, 0u, 0u};
   const typename M::ptr ra = M::add(a, (int32_t)my_off);

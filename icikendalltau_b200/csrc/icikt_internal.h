@@ -61,6 +61,7 @@ struct TiledShape {
   int inplace_kk = 0;    // != 0: in-place variant for long vectors (one sequence buffer, kk fixed at compile time)
   bool gmem = false;     // region lives in the global scratch (does not fit shared memory)
   bool const_gmem = false;  // same for the per-column constant kernel
+  bool radix = false;    // pass A's levels below the top bits are radix-16 levels (decided by n alone: cconst depends on it)
   int max_ctas = 0;      // CTAs the scratch must provide for
   // filled in by the plan once the scratch exists: bytes per CTA slot and number of slots
   int scratch_stride = 0;

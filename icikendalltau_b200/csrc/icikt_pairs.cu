@@ -1030,6 +1030,7 @@ struct TiledParams {
   long long n_units;
   int n, n32, nstride, wstride;
   int kk;  // pass A: 8-key runs per thread (odd); a warp covers 8*kk 32-element chunks
+  bool radix;  // pass A: radix-16 levels, counter area behind the two sequence buffers (TiledShape::radix)
   // the launch runs only if K1's device-side maxima (any large tie group, most large groups,
   // most distinct values of a column) select its tier: lets the host enqueue the shapes of all
   // tiers back to back without reading anything back
@@ -1226,6 +1227,9 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
   constexpr int AQ = IP != 0 ? 2 : 4;  // bytes of the pass-A buffers in units of cap
   // in place: the rank table passes through the counter area in parts, the first group is sorted with the large ones
   constexpr bool STG = IP != 0;
+  // pass A's radix-16 levels (TiledParams::radix) are compiled into the roomy register class only: in the tighter
+  // ones they spill more, so a radix shape always launches that class (launch_tiled_cls)
+  constexpr bool RX = !G && IP == 0 && MAXT == 1024 && MINB == 1;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int T = blockDim.x, nwarps = T >> 5;
@@ -1429,7 +1433,7 @@ __global__ void __launch_bounds__(MAXT, MINB) pairs_tiled_kernel(const TiledPara
                                                reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc, accA, lead);
       else
         count_pass<G, CZ>(bufA, bufB16, kk, nwarps, L, sm.descT, reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc,
-                          accA, lead, len);
+                          accA, lead, len, (RX && p.radix) ? sm.region + 4u * (uint32_t)cap : 0u);
       if (IP == 0 && m > 0 && by_pass_b) {
         const int kkB = (((m + 31) >> 5) + nwarps - 1) / nwarps;
         const int capB = (nwarps * kkB) << 5;
@@ -1539,7 +1543,8 @@ __global__ void __launch_bounds__(1024, 1) column_const_kernel(const TiledParams
     for (int q = tid; q < cap; q += T) M::st16(M::add(bufA, q << 1), (q < n) ? (uint32_t)rk[pm[q]] : padA);
     __syncthreads();
     unsigned long long accA = 0;
-    count_pass<G>(bufA, bufB, kk, nwarps, CS.levels, sm.descT, reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc, accA);
+    count_pass<G>(bufA, bufB, kk, nwarps, CS.levels, sm.descT, reinterpret_cast<uint32_t*>(sm.descB), lane, warp, p.pc, accA,
+                  0u, 0u, (!G && p.radix) ? sm.region + 4u * (uint32_t)cap : 0u);
     const unsigned long long s = warp_sum_u64(accA);
     if (lane == 0) sm.red[warp] = s;
     __syncthreads();
@@ -1844,6 +1849,7 @@ TiledParams make_params(const PairLaunch& pl) {
   p.scratch = nullptr;
   p.scratch_stride = 0;
   p.kk = 0;
+  p.radix = false;
   p.max_tied = t.max_tied;
   p.tier = 0;
   p.budget = 16LL * t.n;
@@ -1911,23 +1917,31 @@ static int const_warps(int64_t n) {
   return W;
 }
 
+// Pass A's radix-16 levels (count_pass, radix_level) need, behind the two sequence buffers, a u16 slot counter per
+// digit and thread (plus the 64 bytes its odd threads' last row runs over) and 32 bytes of node totals per warp
+static int radix_area_bytes(int W) { return 16 * 2 * 32 * W + 64 + 32 * W; }
+// region of the per-column constant kernel: its two sequence buffers and, with radix levels, their counter area
+static int const_region(int64_t n, int W, bool radix) {
+  return (2 * 2 * (W * odd_runs(n, W) * 256) + (radix ? radix_area_bytes(W) : 0) + 15) & ~15;
+}
+
 // Launch shape for vectors of length n: warps per CTA, 8-key runs per thread (odd), bytes of the
 // ping-pong region (pass A: two u16 buffers; pass B: two u32 buffers sized for the largest tied
 // list), and whether the region fits shared memory or has to live in the global scratch.
-TiledShape tiled_shape(int64_t n, int tier, int64_t wstride, int n_sm, int64_t n_units, bool allow_inplace) {
+// `radix`: pass A runs radix-16 levels, the region holds their counter area behind the two buffers.
+static TiledShape shape_for(int64_t n, int tier, int64_t wstride, int n_sm, int64_t n_units, bool allow_inplace,
+                            bool radix) {
   TiledShape sh;
-  auto smem_with = [&](int w, int quarters) {
-    const int cap = w * odd_runs(n, w) * 256;
-    return tiled_smem_bytes((quarters * cap + 15) & ~15, (int)wstride, fmask_words(w, odd_runs(n, w) << 3));
-  };
+  sh.radix = radix;
   // pass A: two u16 buffers (4*cap bytes).  Tier 1 adds a quarter more (cap bytes) for the rank
   // counters of the large tie groups -- a larger counter area means fewer rounds over the large
   // groups but fewer CTAs per SM, which measured worse (profiles/).  Tier 2: twice as much for
-  // pass B's two u32 buffers.
+  // pass B's two u32 buffers.  The radix levels' counters use what lies behind the two buffers
+  // (free during pass A) and extend the region where that is too small.
   auto quarters_of = [&](int) { return tier == 0 ? 4 : tier == 1 ? 5 : 8; };
   auto region_of = [&](int w) {
     const int cap = w * odd_runs(n, w) * 256;
-    return (quarters_of(w) * cap + 15) & ~15;
+    return (std::max(quarters_of(w) * cap, radix ? 4 * cap + radix_area_bytes(w) : 0) + 15) & ~15;
   };
   auto smem_of = [&](int w) {
     return tiled_smem_bytes(region_of(w), (int)wstride, fmask_words(w, odd_runs(n, w) << 3));
@@ -1986,13 +2000,31 @@ TiledShape tiled_shape(int64_t n, int tier, int64_t wstride, int n_sm, int64_t n
   }
   {  // the per-column constant kernel has its own shape: its pass-A buffers must fit a scratch slot too
     const int Wc = const_warps(n);
-    sh.const_region_bytes = (2 * 2 * (Wc * odd_runs(n, Wc) * 256) + 15) & ~15;
+    sh.const_region_bytes = const_region(n, Wc, radix);
     sh.const_gmem = tiled_smem_bytes(sh.const_region_bytes, (int)wstride, fmask_words(Wc, odd_runs(n, Wc) << 3)) > 227 * 1024 ||
                     getenv("ICIKT_FORCE_GMEM") != nullptr;
   }
   sh.gmem = sh.inplace_kk == 0 && (smem_of(W) > 227 * 1024 || getenv("ICIKT_FORCE_GMEM") != nullptr);
   sh.max_ctas = n_sm * std::max(1, 2048 / (32 * W));
   return sh;
+}
+
+// Pass A's level structure is part of every column's constant cconst, so it follows from n alone, the same
+// for all three tiers and the constant kernel: radix-16 levels where each of them runs the two-buffer kernel
+// in shared memory with the counter area, above the lengths the fused column kernel covers (its pass keeps
+// the two-bit levels).  The tuning knobs that pin a shape (ICIKT_WARPS, ICIKT_FORCE_GMEM) act in shape_for, so
+// a pinned shape that leaves shared memory keeps the two-bit levels for every tier.
+static bool pass_a_radix(int64_t n, int64_t wstride) {
+  if (n <= 8192) return false;
+  for (int tier = 0; tier <= 2; ++tier) {
+    const TiledShape sh = shape_for(n, tier, wstride, 1, 0, true, true);
+    if (sh.gmem || sh.inplace_kk != 0 || sh.const_gmem) return false;
+  }
+  return true;
+}
+
+TiledShape tiled_shape(int64_t n, int tier, int64_t wstride, int n_sm, int64_t n_units, bool allow_inplace) {
+  return shape_for(n, tier, wstride, n_sm, n_units, allow_inplace, pass_a_radix(n, wstride));
 }
 
 namespace {
@@ -2063,9 +2095,9 @@ int launch_tiled_cls(const TiledParams& p, const TiledShape& sh, size_t smem, in
   const int o32 = tiled_occupancy<1024, 2, G, false, 0, CZ>(threads, smem);
   // the tighter classes spill: they have to buy at least a quarter more resident CTAs
   int cls = 0, best = o64;
-  if (4 * o40 >= 5 * best) { cls = 1; best = o40; }
-  if (4 * o32 >= 5 * best) { cls = 2; best = o32; }
-  if (const char* e = getenv("ICIKT_REGCLASS")) {
+  if (!p.radix && 4 * o40 >= 5 * best) { cls = 1; best = o40; }
+  if (!p.radix && 4 * o32 >= 5 * best) { cls = 2; best = o32; }
+  if (const char* e = getenv("ICIKT_REGCLASS"); e && !p.radix) {
     const int v = atoi(e);
     if (v == 0 && o64 > 0) { cls = 0; best = o64; }
     if (v == 1 && o40 > 0) { cls = 1; best = o40; }
@@ -2091,6 +2123,7 @@ int launch_pairs_tiled(const PairLaunch& pl, const TiledShape& sh, int n_sm, int
   p.tier = tier;
   p.kk = sh.kk;
   p.region_bytes = sh.region_bytes;
+  p.radix = sh.radix;
   p.scratch = pl.scratch;
   p.scratch_stride = sh.scratch_stride;
   const int fw = fmask_words(sh.warps, sh.kk << 3);
@@ -2108,8 +2141,8 @@ int launch_column_consts(ColumnTables& tab, const TiledShape& sh, unsigned char*
   TiledParams p = make_params(pl);
   const int W = const_warps(tab.n);
   p.kk = odd_runs(tab.n, W);
-  const int cap = W * p.kk * 256;
-  const int region = (2 * 2 * cap + 15) & ~15;
+  p.radix = sh.radix;
+  const int region = const_region(tab.n, W, sh.radix);
   const int fw = fmask_words(W, p.kk << 3);
   const bool g = tiled_smem_bytes(region, p.wstride, fw) > 227 * 1024 || getenv("ICIKT_FORCE_GMEM") != nullptr;
   long long grid = col_hi - col_lo;

@@ -671,8 +671,9 @@ int64_t icikt_stage_table(int64_t C, int32_t include_diag, int32_t cta_slots, in
  * in icikt_plan_columns): tier 0 / 1 / 2 = no large tie groups / large groups sorted in place / pass B.
  * out[0] warps per CTA, out[1] 8-key runs per thread, out[2] bytes of the per-CTA region (sequence buffers +
  * counter area), out[3] variant (0 two sequence buffers in shared memory, 1 in place, 2 global scratch),
- * out[4] padded length (keys), out[5] in place: rows per staging part of the gather.  n_sm = SMs of the device
- * (148), complete_obs != 0 for the complete-observations mode.                                            */
+ * out[4] padded length (keys), out[5] in place: rows per staging part of the gather, out[6] 1 if pass A runs
+ * radix-16 levels below its top bits (chosen by n alone).  n_sm = SMs of the device (148), complete_obs != 0
+ * for the complete-observations mode.                                                                     */
 int icikt_launch_shape(int64_t n, int32_t tier, int32_t n_sm, int32_t complete_obs, int32_t* out);
 
 /* Measures the shared-memory bandwidth of `device` with a conflict-free read+write sweep
