@@ -48,7 +48,8 @@ EXPORTS = [
     "icikt_p_adjust", "icikt_all_pairs_edges_padj", "icikt_all_pairs_edges_padj_multi", "icikt_cross_edges_padj",
     "icikt_cross_edges_padj_multi", "icikt_edges_copy_padj", "icikt_edges_n_tests",
     "icikt_all_pairs_count_edges", "icikt_all_pairs_count_edges_multi", "icikt_cross_count_edges",
-    "icikt_cross_count_edges_multi",
+    "icikt_cross_count_edges_multi", "icikt_all_pairs_components", "icikt_all_pairs_components_multi",
+    "icikt_cross_components", "icikt_cross_components_multi",
 ]
 NSTATUS = 10
 
@@ -237,6 +238,13 @@ def load():
     cnt = [ctypes.POINTER(EdgeFilter), ctypes.c_int32, _lp]
     tail = [_lp, _dp, ctypes.POINTER(Timings)]
     for name, lead, deg in (("icikt_all_pairs_count_edges", one, [_lp]), ("icikt_cross_count_edges", cross, [_lp, _lp])):
+        getattr(L, name).argtypes = lead + cnt + deg + tail
+        getattr(L, name + "_multi").argtypes = lead + [_ip, ctypes.c_int32] + cnt + deg + tail
+        getattr(L, name).restype = getattr(L, name + "_multi").restype = ctypes.c_int
+    # the component calls: the count calls' arguments with (component or x_component + y_component, n_components)
+    # after the degrees
+    for name, lead, deg in (("icikt_all_pairs_components", one, [_lp, _ip, _lp]),
+                            ("icikt_cross_components", cross, [_lp, _lp, _ip, _ip, _lp])):
         getattr(L, name).argtypes = lead + cnt + deg + tail
         getattr(L, name + "_multi").argtypes = lead + [_ip, ctypes.c_int32] + cnt + deg + tail
         getattr(L, name).restype = getattr(L, name + "_multi").restype = ctypes.c_int
@@ -641,13 +649,16 @@ def _count_filters(filters):
     return arr, len(fl)
 
 
-def run_count_edges(data, global_na=(), filters=((None, None),), devices=None, want_degree=True, **opt_kw):
+def run_count_edges(data, global_na=(), filters=((None, None),), devices=None, want_degree=True,
+                    want_components=False, **opt_kw):
     """icikt_all_pairs_count_edges: for every filter (min_abs_cor, max_pvalue) of `filters` (None: no bound), the
     number of pairs that pass it -- exactly the rows run_edges(..., scale_max=False) returns with that filter -- and
     every column's degree among them, in one walk of the pair order; no pair comes back.  data may be a scipy.sparse
     matrix.  devices: list of CUDA ordinals -> icikt_all_pairs_count_edges_multi, bit for bit the single-device
     result.  Returns a dict with n_pass (T,) int64, degree (C, T) int64 (a diagonal pair counts once; None without
-    want_degree), status_counts (NSTATUS,) int64 (pairs per status class), max_taumax and timings."""
+    want_degree), status_counts (NSTATUS,) int64 (pairs per status class), max_taumax and timings.
+    want_components -> icikt_all_pairs_components in the same walk: the dict adds component (C, T) int32, the
+    smallest column of the column's connected component under each filter, and n_components (T,) int64."""
     L = load()
     arr, T = _count_filters(filters)
     xi, n, C, keep_alive = _input(data)
@@ -659,17 +670,29 @@ def run_count_edges(data, global_na=(), filters=((None, None),), devices=None, w
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
+    if want_components:
+        comp = np.zeros((C, max(T, 1)), dtype=np.int32)
+        ncomp = np.zeros(max(T, 1), dtype=np.int64)
+        check(getattr(L, "icikt_all_pairs_components" + msfx)(ctypes.byref(xi), n, gp, ng, ctypes.byref(o), *dargs,
+                                                              arr, T, _ptr(n_pass), _ptr(degree), _ptr(comp),
+                                                              _ptr(ncomp), _ptr(hist), ctypes.byref(mx),
+                                                              ctypes.byref(t)))
+        return dict(n_pass=n_pass, degree=degree, component=comp, n_components=ncomp, status_counts=hist,
+                    max_taumax=mx.value, timings=t.as_dict())
     check(getattr(L, "icikt_all_pairs_count_edges" + msfx)(ctypes.byref(xi), n, gp, ng, ctypes.byref(o), *dargs, arr,
                                                            T, _ptr(n_pass), _ptr(degree), _ptr(hist), ctypes.byref(mx),
                                                            ctypes.byref(t)))
     return dict(n_pass=n_pass, degree=degree, status_counts=hist, max_taumax=mx.value, timings=t.as_dict())
 
 
-def run_cross_count_edges(x, y, global_na=(), filters=((None, None),), devices=None, want_degree=True, **opt_kw):
+def run_cross_count_edges(x, y, global_na=(), filters=((None, None),), devices=None, want_degree=True,
+                          want_components=False, **opt_kw):
     """icikt_cross_count_edges: run_count_edges over the cross order of x against y (the rows run_cross_edges(...,
     scale_max=False) returns).  devices -> icikt_cross_count_edges_multi, bit for bit the single-device result.
     Returns a dict with n_pass (T,), x_degree (Cx, T), y_degree (Cy, T) (None without want_degree), status_counts,
-    max_taumax and timings."""
+    max_taumax and timings.  want_components -> icikt_cross_components: the dict adds x_component (Cx, T) and
+    y_component (Cy, T) int32, labels that index the columns of [x | y] (y's column j is Cx + j), and n_components
+    (T,) int64."""
     L = load()
     arr, T = _count_filters(filters)
     xi, yi, n, cx, cy, keep_alive = _cross_inputs(x, y)
@@ -682,6 +705,16 @@ def run_cross_count_edges(x, y, global_na=(), filters=((None, None),), devices=N
     mx = ctypes.c_double(float("nan"))
     t = Timings()
     g, gp, ng = _global_na_array(global_na)
+    if want_components:
+        xc = np.zeros((cx, max(T, 1)), dtype=np.int32)
+        yc = np.zeros((cy, max(T, 1)), dtype=np.int32)
+        ncomp = np.zeros(max(T, 1), dtype=np.int64)
+        check(getattr(L, "icikt_cross_components" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng,
+                                                          ctypes.byref(o), *dargs, arr, T, _ptr(n_pass), _ptr(xd),
+                                                          _ptr(yd), _ptr(xc), _ptr(yc), _ptr(ncomp), _ptr(hist),
+                                                          ctypes.byref(mx), ctypes.byref(t)))
+        return dict(n_pass=n_pass, x_degree=xd, y_degree=yd, x_component=xc, y_component=yc, n_components=ncomp,
+                    status_counts=hist, max_taumax=mx.value, timings=t.as_dict())
     check(getattr(L, "icikt_cross_count_edges" + msfx)(ctypes.byref(xi), ctypes.byref(yi), n, gp, ng, ctypes.byref(o),
                                                        *dargs, arr, T, _ptr(n_pass), _ptr(xd), _ptr(yd), _ptr(hist),
                                                        ctypes.byref(mx), ctypes.byref(t)))

@@ -596,7 +596,7 @@ def _count_grid(min_abs_cor, max_pvalue):
 
 def ici_kendalltau_edge_counts(data_matrix, min_abs_cor=None, max_pvalue=None, global_na=(np.nan, np.inf, 0),
                                perspective="global", diag_good=True, alternative="two.sided", continuity=False,
-                               colnames=None, device=0, n_gpus=1):
+                               colnames=None, device=0, n_gpus=1, components=False):
     """How many rows ici_kendalltau(..., return_matrix=False, scale_max=False, min_abs_cor=t, max_pvalue=p) would
     return, and each sample's degree among them, for a whole grid of thresholds in one pass over the pairs -- the
     counts a network threshold is chosen from, without the rows.
@@ -613,6 +613,11 @@ def ici_kendalltau_edge_counts(data_matrix, min_abs_cor=None, max_pvalue=None, g
     Returns a dict with `n_edges` (int64, the grid's shape: () for two scalars), `degree` (C x the grid's shape:
     the rows that have the sample as s1 or s2, a diagonal row counting once), `names`, `min_abs_cor`, `max_pvalue`
     (the grid's bounds), `max_taumax` and `run_time`.
+
+    components=True adds, in the same pass, the connected components of each threshold's network of samples:
+    `component` (C x the grid's shape, int32: the index in `names` of the first sample of the sample's component; a
+    sample without an edge is its own component), `n_components` and `largest_component` (the grid's shape, int64).
+    diag_good's diagonal rows are self-loops and change no component.
     """
     filters, shape = _count_grid(min_abs_cor, max_pvalue)
     data, names = _colnames_of(data_matrix, colnames, "data_matrix")
@@ -626,7 +631,7 @@ def ici_kendalltau_edge_counts(data_matrix, min_abs_cor=None, max_pvalue=None, g
         kw["devices"] = range(n_gpus)
     log.info("Counting edges ...")
     t1 = time.perf_counter()
-    r = _lib.run_count_edges(data, global_na, filters, include_diag=not diag_good, **kw)
+    r = _lib.run_count_edges(data, global_na, filters, include_diag=not diag_good, want_components=components, **kw)
     run_time = time.perf_counter() - t1
     _warn_status_counts(r["status_counts"])
     n_edges, degree = r["n_pass"], r["degree"]
@@ -638,13 +643,29 @@ def ici_kendalltau_edge_counts(data_matrix, min_abs_cor=None, max_pvalue=None, g
             sel = _edge_mask(dg, dp, t, p)
             n_edges[f] += int(sel.sum())
             degree[sel, f] += 1
-    return dict(n_edges=n_edges.reshape(shape), degree=degree.reshape((C,) + shape), names=names,
-                min_abs_cor=min_abs_cor, max_pvalue=max_pvalue, max_taumax=r["max_taumax"], run_time=run_time)
+    out = dict(n_edges=n_edges.reshape(shape), degree=degree.reshape((C,) + shape), names=names,
+               min_abs_cor=min_abs_cor, max_pvalue=max_pvalue, max_taumax=r["max_taumax"], run_time=run_time)
+    if components:
+        out.update(_components_of(r, (r["component"],), shape))
+    return out
+
+
+def _components_of(r, labels, shape):
+    """`component` (or `x_component`, `y_component`), `n_components` and `largest_component` of a component call's
+    result r, whose label tables `labels` cover every vertex once, reshaped to the grid"""
+    lab = np.concatenate(labels)
+    largest = np.array([np.bincount(lab[:, f]).max() for f in range(lab.shape[1])], dtype=np.int64)
+    out = dict(n_components=r["n_components"].reshape(shape), largest_component=largest.reshape(shape))
+    if len(labels) == 1:
+        out["component"] = labels[0].reshape((labels[0].shape[0],) + shape)
+    else:
+        out["x_component"], out["y_component"] = (v.reshape((v.shape[0],) + shape) for v in labels)
+    return out
 
 
 def ici_kendalltau_cross_edge_counts(x, y, min_abs_cor=None, max_pvalue=None, global_na=(np.nan, np.inf, 0),
                                      perspective="global", alternative="two.sided", continuity=False, xnames=None,
-                                     ynames=None, device=0, n_gpus=1):
+                                     ynames=None, device=0, n_gpus=1, components=False):
     """ici_kendalltau_edge_counts for the pairs of x's samples with y's: how many rows
     ici_kendalltau_cross(x, y, return_matrix=False, scale_max=False, min_abs_cor=t, max_pvalue=p) would return, for
     the grid of min_abs_cor x max_pvalue, counted on the device (_lib.run_cross_count_edges).  n_gpus > 1 spreads
@@ -653,6 +674,11 @@ def ici_kendalltau_cross_edge_counts(x, y, min_abs_cor=None, max_pvalue=None, gl
     Returns a dict with `n_edges` (the grid's shape), `x_degree` (Cx x the grid's shape: rows with x's sample as
     s1), `y_degree` (Cy x the grid's shape: rows with y's sample as s2), `xnames`, `ynames`, `min_abs_cor`,
     `max_pvalue`, `max_taumax` and `run_time`.
+
+    components=True adds the connected components of each threshold's network over the samples of x and y together:
+    `x_component` (Cx x the grid's shape) and `y_component` (Cy x the grid's shape), int32 indices into
+    xnames + ynames of the first sample of each sample's component, `n_components` and `largest_component` (the
+    grid's shape).
     """
     filters, shape = _count_grid(min_abs_cor, max_pvalue)
     x, y, xnames, ynames = _cross_data(x, y, xnames, ynames)
@@ -662,12 +688,15 @@ def ici_kendalltau_cross_edge_counts(x, y, min_abs_cor=None, max_pvalue=None, gl
         kw["devices"] = range(n_gpus)
     log.info("Counting edges ...")
     t1 = time.perf_counter()
-    r = _lib.run_cross_count_edges(x, y, global_na, filters, **kw)
+    r = _lib.run_cross_count_edges(x, y, global_na, filters, want_components=components, **kw)
     run_time = time.perf_counter() - t1
     _warn_status_counts(r["status_counts"])
-    return dict(n_edges=r["n_pass"].reshape(shape), x_degree=r["x_degree"].reshape((x.shape[1],) + shape),
-                y_degree=r["y_degree"].reshape((y.shape[1],) + shape), xnames=xnames, ynames=ynames,
-                min_abs_cor=min_abs_cor, max_pvalue=max_pvalue, max_taumax=r["max_taumax"], run_time=run_time)
+    out = dict(n_edges=r["n_pass"].reshape(shape), x_degree=r["x_degree"].reshape((x.shape[1],) + shape),
+               y_degree=r["y_degree"].reshape((y.shape[1],) + shape), xnames=xnames, ynames=ynames,
+               min_abs_cor=min_abs_cor, max_pvalue=max_pvalue, max_taumax=r["max_taumax"], run_time=run_time)
+    if components:
+        out.update(_components_of(r, (r["x_component"], r["y_component"]), shape))
+    return out
 
 
 _NA_METHODS = ("all.obs", "complete.obs", "pairwise.complete.obs", "everything", "na.or.complete")

@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libicikt_b200.so")
 SOURCES = ["icikt_capi.cu", "icikt_columns.cu", "icikt_pairs.cu", "icikt_padj.cu", "icikt_reshape.cu", "icikt_select.cu"]
-HEADERS = ["icikt_common.cuh", "icikt_count.cuh", "icikt_cross.cuh", "icikt_edges.cuh", "icikt_internal.h", "icikt_owned.h", "icikt_padj.cuh", "icikt_topk.cuh", os.path.join("..", "..", "include", "icikt_b200.h")]
+HEADERS = ["icikt_common.cuh", "icikt_components.cuh", "icikt_count.cuh", "icikt_cross.cuh", "icikt_edges.cuh", "icikt_internal.h", "icikt_owned.h", "icikt_padj.cuh", "icikt_topk.cuh", os.path.join("..", "..", "include", "icikt_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
     "--fmad=false",  # keep the fp64 epilogue's operation order (no contraction)

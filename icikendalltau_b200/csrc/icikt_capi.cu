@@ -20,6 +20,7 @@
 #include <vector>
 
 #include "../../include/icikt_b200.h"
+#include "icikt_components.cuh"
 #include "icikt_cross.cuh"
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
@@ -295,8 +296,10 @@ struct icikt_plan {
   DeviceArray<int32_t> d_midx;   // [entries]
   DeviceArray<double> d_mlist;   // 4 x [entries]: raw, pvalue, taumax, completeness
   // Edge-count calls (icikt_all_pairs_count_edges), summed over the windows: [16] pairs per status class, [T] passing
-  // pairs per filter, then, if degrees are wanted, [T][C] degrees (filter-major)
+  // pairs per filter, then, if degrees are wanted, [T][C] degrees (filter-major), then, for the component calls, [T]
+  // successful hooks; d_eparent holds their [T][C] union-find forests (icikt_components.cuh)
   DeviceArray<unsigned long long> d_ecount;
+  DeviceArray<int32_t> d_eparent;
 
   Event ev[9];
   icikt_timings tm{};
@@ -2048,6 +2051,7 @@ struct CountSpec {
   int T = 0;
   double t[kCountFiltersMax], a[kCountFiltersMax];  // min_abs_cor, max_pvalue of every filter (NaN: no condition)
   bool degree = false;                              // the caller wants degrees
+  bool components = false;                          // the component calls: forests, hooks and labels
 };
 
 // one of the caller's degree tables: plan columns [c_lo, c_hi), entry (c - c_lo) * T + f (may be null)
@@ -2056,16 +2060,34 @@ struct DegreeOut {
   int64_t c_lo, c_hi;
 };
 
+// one of the caller's label tables, in the layout of DegreeOut
+struct ComponentOut {
+  int32_t* out;
+  int64_t c_lo, c_hi;
+};
+
 // The edge-count walk over pairs [first, last) of `order`: the counters start at zero and every window's tally adds
-// to them; then they come back once into `out` (d_ecount's layout) and d2h_ms receives the time of that copy.
+// to them; then they come back once into `out` (d_ecount's layout) and d2h_ms receives the time of that copy.  With
+// cs.components the tally also unites each filter's forest, whose labels (the kernel that resolves them included in
+// d2h_ms) come back into `labels`, [T][C] filter-major.  The forest is set to parent[v] = v just before the first
+// window's tally, on the same stream, so that its time counts in epilogue_ms with the tally's.
 template <class Order>
 static int count_walk(icikt_plan* p, const Order& order, const CountSpec& cs, int64_t first, int64_t last, int64_t W,
-                      WalkTotals& tot, std::vector<unsigned long long>& out, float& d2h_ms) {
-  const size_t entries = 16 + (size_t)cs.T + (cs.degree ? (size_t)cs.T * (size_t)p->C : 0);
+                      WalkTotals& tot, std::vector<unsigned long long>& out, std::vector<int32_t>& labels,
+                      float& d2h_ms) {
+  const size_t hooks_at = 16 + (size_t)cs.T + (cs.degree ? (size_t)cs.T * (size_t)p->C : 0);
+  const size_t entries = hooks_at + (cs.components ? (size_t)cs.T : 0);
+  const size_t n_labels = cs.components ? (size_t)cs.T * (size_t)p->C : 0;
   ECK(p->d_ecount.reserve(entries));
   unsigned long long* c = p->d_ecount.get();
   CK(cudaMemsetAsync(c, 0, sizeof(unsigned long long) * entries, p->stream));
-  auto select = [&](int64_t, int, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
+  if (cs.components) ECK(p->d_eparent.reserve(n_labels));
+  auto select = [&](int64_t w, int, const PairUnit* units, int64_t n_units, int64_t n_slots) -> int {
+    if (cs.components && w == 0) {
+      const int l = launch_component_init(p->d_eparent.get(), cs.T, p->C, p->stream);
+      if (l < 0) return launch_fail("component init kernel");
+      tot.launches += l;
+    }
     EdgeTally et;
     et.units = units;
     et.n_units = n_units;
@@ -2080,6 +2102,8 @@ static int count_walk(icikt_plan* p, const Order& order, const CountSpec& cs, in
     et.status_counts = c;
     et.n_pass = c + 16;
     et.degree = cs.degree ? c + 16 + cs.T : nullptr;
+    et.parent = cs.components ? p->d_eparent.get() : nullptr;
+    et.hooks = cs.components ? c + hooks_at : nullptr;
     const int l = launch_edge_tally(et, p->stream);
     if (l < 0) return launch_fail("edge tally kernel");
     tot.launches += l;
@@ -2089,11 +2113,19 @@ static int count_walk(icikt_plan* p, const Order& order, const CountSpec& cs, in
   if (rc != ICIKT_OK) return rc;
   try {
     out.resize(entries);
+    labels.resize(n_labels);
   } catch (const std::bad_alloc&) {
     return fail(ICIKT_ERR_ALLOC, "out of host memory for the counters");
   }
   CK(cudaEventRecord(p->ev[6], p->stream));
+  if (cs.components) {
+    const int l = launch_component_labels(p->d_eparent.get(), cs.T, p->C, p->stream);
+    if (l < 0) return launch_fail("component labels kernel");
+    tot.launches += l;
+  }
   rc = staged_copy_out(p, out.data(), c, sizeof(unsigned long long) * entries, p->stream);
+  if (rc == ICIKT_OK && n_labels)
+    rc = staged_copy_out(p, labels.data(), p->d_eparent.get(), sizeof(int32_t) * n_labels, p->stream);
   if (rc != ICIKT_OK) return rc;
   CK(cudaEventRecord(p->ev[7], p->stream));
   CK(cudaEventSynchronize(p->ev[7]));
@@ -3271,12 +3303,15 @@ int check_count_filters(const icikt_edge_filter* filters, int32_t n_filters, con
 
 // The counting job over the devices of J, its arguments checked: every worker walks its slice with its own counters,
 // and the host sums them into the caller's arrays (integers: the sum is that of one device).  deg: the caller's
-// degree tables, each over plan columns [c_lo, c_hi).
+// degree tables, each over plan columns [c_lo, c_hi).  With cs.components, comp receives the labels in the same way
+// and n_components (may be null) their count: one device's labels as they are, several devices' merged on the host.
 int count_run(MultiJob& J, const CountSpec& cs, int64_t* n_pass, const std::vector<DegreeOut>& deg,
-              int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+              int64_t* status_counts, double* max_taumax, icikt_timings* timings,
+              const std::vector<ComponentOut>& comp = {}, int64_t* n_components = nullptr) {
   int rc = select_device(J.device_of(0));
   if (rc != ICIKT_OK) return rc;
   std::vector<std::vector<unsigned long long>> got((size_t)J.n_devices);
+  std::vector<std::vector<int32_t>> labels((size_t)J.n_devices);
   std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
   if (J.ptot > 0) {
     std::vector<MultiWork> work;
@@ -3292,7 +3327,7 @@ int count_run(MultiJob& J, const CountSpec& cs, int64_t* n_pass, const std::vect
       r = ensure_walk_buffers(p);
       if (r == ICIKT_OK)
         r = with_order(J, p, [&](const auto& order) {
-          return count_walk(p, order, cs, lo, hi, p->P, tot, got[(size_t)k], d2h_ms);
+          return count_walk(p, order, cs, lo, hi, p->P, tot, got[(size_t)k], labels[(size_t)k], d2h_ms);
         });
       if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
       bits[(size_t)k] = tot.bits;
@@ -3318,16 +3353,48 @@ int count_run(MultiJob& J, const CountSpec& cs, int64_t* n_pass, const std::vect
       for (int64_t c = d.c_lo; c < d.c_hi; ++c)
         for (int f = 0; f < T; ++f) d.out[(c - d.c_lo) * T + f] = sum(16 + (size_t)T + (size_t)f * (size_t)C + (size_t)c);
   if (J.ptot > 0 && max_taumax) *max_taumax = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  if (!cs.components) return ICIKT_OK;
+  std::vector<const int32_t*> walked;  // the devices that walked pairs
+  const std::vector<unsigned long long>* hooks = nullptr;
+  for (size_t k = 0; k < labels.size(); ++k)
+    if (!labels[k].empty()) {
+      walked.push_back(labels[k].data());
+      hooks = &got[k];
+    }
+  std::vector<int32_t> merged;
+  std::vector<int64_t> count((size_t)T);
+  const int32_t* lab = walked.empty() ? nullptr : walked[0];
+  if (walked.size() == 1) {  // V - hooks: every successful hook joined two trees
+    const size_t hooks_at = 16 + (size_t)T + (cs.degree ? (size_t)T * (size_t)C : 0);
+    for (int f = 0; f < T; ++f) count[(size_t)f] = C - (int64_t)(*hooks)[hooks_at + (size_t)f];
+  } else {  // several slices, or none (no pairs: every vertex alone)
+    try {
+      merged.resize((size_t)T * (size_t)C);
+    } catch (const std::bad_alloc&) {
+      return fail(ICIKT_ERR_ALLOC, "out of host memory for the labels");
+    }
+    merge_component_labels(T, C, walked, merged.data(), count.data());
+    lab = merged.data();
+  }
+  for (const ComponentOut& d : comp)
+    if (d.out)
+      for (int64_t c = d.c_lo; c < d.c_hi; ++c)
+        for (int f = 0; f < T; ++f) d.out[(c - d.c_lo) * T + f] = lab[(size_t)f * (size_t)C + (size_t)c];
+  if (n_components) std::copy(count.begin(), count.end(), n_components);
   return ICIKT_OK;
 }
 
+// components: the component calls, whose `component` is required (the count calls pass false and nulls)
 int count_edges_impl(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na, const icikt_opts& o,
                      const int32_t* devices, int32_t n_devices, const icikt_edge_filter* filters, int32_t n_filters,
                      int64_t* n_pass, int64_t* degree, int64_t* status_counts, double* max_taumax,
-                     icikt_timings* timings) {
+                     icikt_timings* timings, bool components = false, int32_t* component = nullptr,
+                     int64_t* n_components = nullptr) {
   ColumnSource s;
   CountSpec cs;
   int rc = check_count_filters(filters, n_filters, n_pass, degree != nullptr, &cs);
+  cs.components = components;
+  if (rc == ICIKT_OK && components && !component) rc = fail(ICIKT_ERR_BAD_ARG, "component is NULL");
   if (rc == ICIKT_OK) rc = n < 1 ? fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1") : cross_source(x, "x", n, &s);
   if (rc == ICIKT_OK) rc = check_window_args(s, n, s.C, global_na, n_global_na, o);
   if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
@@ -3335,23 +3402,30 @@ int count_edges_impl(const icikt_input* x, int64_t n, const double* global_na, i
   MultiJob J(n_devices);
   J.src = s; J.n = n; J.C = s.C; J.global_na = global_na; J.n_global_na = n_global_na;
   J.devices = devices; J.base = o; J.ptot = tri_pairs(s.C) + (o.include_diag ? s.C : 0);
-  return count_run(J, cs, n_pass, {DegreeOut{degree, 0, s.C}}, status_counts, max_taumax, timings);
+  return count_run(J, cs, n_pass, {DegreeOut{degree, 0, s.C}}, status_counts, max_taumax, timings,
+                   {ComponentOut{component, 0, s.C}}, n_components);
 }
 
 int cross_count_edges_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
                            int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices,
                            const icikt_edge_filter* filters, int32_t n_filters, int64_t* n_pass, int64_t* x_degree,
-                           int64_t* y_degree, int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+                           int64_t* y_degree, int64_t* status_counts, double* max_taumax, icikt_timings* timings,
+                           bool components = false, int32_t* x_component = nullptr, int32_t* y_component = nullptr,
+                           int64_t* n_components = nullptr) {
   ColumnSource sx, sy;
   CountSpec cs;
   int rc = check_count_filters(filters, n_filters, n_pass, x_degree || y_degree, &cs);
+  cs.components = components;
+  if (rc == ICIKT_OK && components && !x_component && !y_component)
+    rc = fail(ICIKT_ERR_BAD_ARG, "x_component and y_component are both NULL: give at least one");
   if (rc == ICIKT_OK) rc = check_cross_args(x, y, n, global_na, n_global_na, o, false, &sx, &sy);
   if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
   cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, 0, sx.C * sy.C);
   return count_run(J, cs, n_pass, {DegreeOut{x_degree, 0, sx.C}, DegreeOut{y_degree, sx.C, sx.C + sy.C}},
-                   status_counts, max_taumax, timings);
+                   status_counts, max_taumax, timings,
+                   {ComponentOut{x_component, 0, sx.C}, ComponentOut{y_component, sx.C, sx.C + sy.C}}, n_components);
 }
 
 }  // namespace
@@ -3725,6 +3799,46 @@ int icikt_cross_count_edges_multi(const icikt_input* x, const icikt_input* y, in
                                   double* max_taumax, icikt_timings* timings) {
   return cross_count_edges_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filters,
                                 n_filters, n_pass, x_degree, y_degree, status_counts, max_taumax, timings);
+}
+
+int icikt_all_pairs_components(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                               const icikt_opts* opts, const icikt_edge_filter* filters, int32_t n_filters,
+                               int64_t* n_pass, int64_t* degree, int32_t* component, int64_t* n_components,
+                               int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return count_edges_impl(x, n, global_na, n_global_na, o, &o.device, 1, filters, n_filters, n_pass, degree,
+                          status_counts, max_taumax, timings, true, component, n_components);
+}
+
+int icikt_all_pairs_components_multi(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                     const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                     const icikt_edge_filter* filters, int32_t n_filters, int64_t* n_pass,
+                                     int64_t* degree, int32_t* component, int64_t* n_components,
+                                     int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  return count_edges_impl(x, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filters, n_filters,
+                          n_pass, degree, status_counts, max_taumax, timings, true, component, n_components);
+}
+
+int icikt_cross_components(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filters,
+                           int32_t n_filters, int64_t* n_pass, int64_t* x_degree, int64_t* y_degree,
+                           int32_t* x_component, int32_t* y_component, int64_t* n_components,
+                           int64_t* status_counts, double* max_taumax, icikt_timings* timings) {
+  const icikt_opts o = opts_or_default(opts);
+  return cross_count_edges_impl(x, y, n, global_na, n_global_na, o, &o.device, 1, filters, n_filters, n_pass, x_degree,
+                                y_degree, status_counts, max_taumax, timings, true, x_component, y_component,
+                                n_components);
+}
+
+int icikt_cross_components_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                                 int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
+                                 int32_t n_devices, const icikt_edge_filter* filters, int32_t n_filters,
+                                 int64_t* n_pass, int64_t* x_degree, int64_t* y_degree, int32_t* x_component,
+                                 int32_t* y_component, int64_t* n_components, int64_t* status_counts,
+                                 double* max_taumax, icikt_timings* timings) {
+  return cross_count_edges_impl(x, y, n, global_na, n_global_na, opts_or_default(opts), devices, n_devices, filters,
+                                n_filters, n_pass, x_degree, y_degree, status_counts, max_taumax, timings, true,
+                                x_component, y_component, n_components);
 }
 
 int icikt_p_adjust(const double* p, int64_t m, int32_t method, int32_t device, double* out, int64_t* n_tests) {

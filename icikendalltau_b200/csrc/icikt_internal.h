@@ -277,8 +277,16 @@ struct EdgeTally {
   unsigned long long* status_counts;  // device [16]: pairs per status class
   unsigned long long* n_pass;         // device [T]
   unsigned long long* degree;         // device [T C], or null
+  // The component calls: each filter's union-find forest over the C columns (icikt_components.cuh), filter-major
+  // [T][C], and its count of successful hooks [T]; null for the count calls, which then run the kernel without unions.
+  int32_t* parent;
+  unsigned long long* hooks;
 };
 int launch_edge_tally(const EdgeTally& s, cudaStream_t stream);
+// The forests of the component calls: parent[f C + v] = v before the first window (launch_component_init), every
+// entry replaced by its root, the component's smallest vertex, after the last (launch_component_labels).
+int launch_component_init(int32_t* parent, int n_filters, int64_t C, cudaStream_t stream);
+int launch_component_labels(int32_t* parent, int n_filters, int64_t C, cudaStream_t stream);
 
 // R's p.adjust on the device (icikt_padj.cu, arithmetic in icikt_padj.cuh).  Each returns the first CUDA error.
 // counts[0] += the non-NaN values of p[0, n); the keys (padj_key) of those <= bound (NaN: all) are appended at

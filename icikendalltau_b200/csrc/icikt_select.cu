@@ -13,6 +13,7 @@
 // The selection of the top-k call (icikt_all_pairs_topk) follows the edge kernels: per-column buckets of the
 // candidates that beat a column's k-th entry, merged into the column's sorted list (see launch_topk_select).  Over
 // several devices, topk_device_merge_kernel folds the devices' lists of a block of columns into one.
+#include "icikt_components.cuh"
 #include "icikt_edges.cuh"
 #include "icikt_internal.h"
 #include "icikt_topk.cuh"
@@ -166,6 +167,10 @@ __global__ void __launch_bounds__(kSelThreads) edge_scatter_kernel(const EdgeSel
 // one shared atomic per lane and one global atomic per CTA and filter); the row endpoint i is shared by the lanes of a
 // unit and usually by the whole warp, so the lanes with the same i add their count with one atomic (match_any), and
 // the other endpoint j takes one atomic per passing pair and filter.  A diagonal pair (i == j) adds 1 to its column.
+// kUnion (the component calls): after the ballots of a round, each lane unites i and j in the forest of every filter
+// its pair passes (icikt_components.cuh), in a loop with no warp-synchronous intrinsic, since lanes retry for
+// different counts.  A filter already at one component when the CTA starts is skipped: no further edge can change it.
+template <bool kUnion>
 __global__ void __launch_bounds__(kSelThreads) edge_tally_kernel(const EdgeTally s) {
   __shared__ unsigned cta_pass[kCountFiltersMax];
   __shared__ unsigned cta_status[16];
@@ -178,6 +183,17 @@ __global__ void __launch_bounds__(kSelThreads) edge_tally_kernel(const EdgeTally
     const long long first_slot = tile * kEdgeTile;
     const long long last_slot = min((long long)s.n_slots, first_slot + kEdgeTile) - 1;
     unit_range[threadIdx.x] = unit_of(s.units, 0, s.n_units, threadIdx.x ? last_slot : first_slot);
+  }
+  unsigned long long open = 0;  // kUnion: the filters with more than one component
+  if constexpr (kUnion) {
+    __shared__ unsigned open_word[2];
+    if (threadIdx.x < kCountFiltersMax) {
+      const bool more = threadIdx.x < T && s.hooks[threadIdx.x] + 1 < (unsigned long long)s.C;
+      const unsigned w = __ballot_sync(FULL, more);
+      if (lane == 0) open_word[threadIdx.x >> 5] = w;
+    }
+    __syncthreads();
+    open = ((unsigned long long)open_word[1] << 32) | open_word[0];
   }
   __syncthreads();
   const long long ua = unit_range[0], ub = unit_range[1] + 1;
@@ -223,6 +239,12 @@ __global__ void __launch_bounds__(kSelThreads) edge_tally_kernel(const EdgeTally
         if (j != i) atomicAdd(deg + j, 1ull);
       }
     }
+    if constexpr (kUnion) {
+      for (unsigned long long u = i != j ? mask & open : 0; u; u &= u - 1) {
+        const int f = __ffsll((long long)u) - 1;
+        if (uf_unite(s.parent + (long long)f * s.C, i, j)) atomicAdd(s.hooks + f, 1ull);
+      }
+    }
   }
   if (pass_lo) atomicAdd(&cta_pass[lane], pass_lo);
   if (pass_hi) atomicAdd(&cta_pass[lane + 32], pass_hi);
@@ -230,6 +252,23 @@ __global__ void __launch_bounds__(kSelThreads) edge_tally_kernel(const EdgeTally
   if (threadIdx.x < T && cta_pass[threadIdx.x]) atomicAdd(s.n_pass + threadIdx.x, (unsigned long long)cta_pass[threadIdx.x]);
   if (threadIdx.x < 16 && cta_status[threadIdx.x])
     atomicAdd(s.status_counts + threadIdx.x, (unsigned long long)cta_status[threadIdx.x]);
+}
+
+// The forests of the component calls, filter-major [T][C]: every vertex its own root before the first window
+__global__ void __launch_bounds__(kSelThreads) component_init_kernel(int32_t* parent, long long n, long long C) {
+  const long long k = (long long)blockIdx.x * kSelThreads + threadIdx.x;
+  if (k < n) parent[k] = (int32_t)(k % C);
+}
+
+// After the last window, every entry becomes its root, the smallest vertex of its component.  The find only reads:
+// a path-halving find could write a grandparent over a root another thread has just stored.  The entries still
+// change under the reads, but only ever to an ancestor, so every walk ends at the same root.
+__global__ void __launch_bounds__(kSelThreads) component_labels_kernel(int32_t* parent, long long n, long long C) {
+  const long long k = (long long)blockIdx.x * kSelThreads + threadIdx.x;
+  if (k >= n) return;
+  int32_t* forest = parent + (k / C) * C;
+  const int32_t v = (int32_t)(k % C);
+  uf_store(forest + v, uf_root(forest, v));
 }
 
 // Top-k: the count pass (kScatter false) and the scatter pass (true) of one tile of kEdgeTile slots.  Both make
@@ -483,7 +522,24 @@ int launch_edge_tally(const EdgeTally& s, cudaStream_t stream) {
   const long long tiles = (s.n_slots + kEdgeTile - 1) / kEdgeTile;
   if (tiles > 0x7fffffffLL || s.n_filters < 1 || s.n_filters > kCountFiltersMax || s.C > 0x7fffffffLL)
     return launch_refused("edge tally: bad arguments");
-  edge_tally_kernel<<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  if (s.parent)
+    edge_tally_kernel<true><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  else
+    edge_tally_kernel<false><<<(unsigned)tiles, kSelThreads, 0, stream>>>(s);
+  return launch_status(1);
+}
+
+int launch_component_init(int32_t* parent, int n_filters, int64_t C, cudaStream_t stream) {
+  const long long n = (long long)n_filters * C, blocks = (n + kSelThreads - 1) / kSelThreads;
+  if (n <= 0 || C > 0x7fffffffLL || blocks > 0x7fffffffLL) return launch_refused("component init: bad arguments");
+  component_init_kernel<<<(unsigned)blocks, kSelThreads, 0, stream>>>(parent, n, C);
+  return launch_status(1);
+}
+
+int launch_component_labels(int32_t* parent, int n_filters, int64_t C, cudaStream_t stream) {
+  const long long n = (long long)n_filters * C, blocks = (n + kSelThreads - 1) / kSelThreads;
+  if (n <= 0 || C > 0x7fffffffLL || blocks > 0x7fffffffLL) return launch_refused("component labels: bad arguments");
+  component_labels_kernel<<<(unsigned)blocks, kSelThreads, 0, stream>>>(parent, n, C);
   return launch_status(1);
 }
 

@@ -574,6 +574,47 @@ int icikt_cross_count_edges_multi(const icikt_input* x, const icikt_input* y, in
                                   int64_t* n_pass, int64_t* x_degree, int64_t* y_degree, int64_t* status_counts,
                                   double* max_taumax, icikt_timings* timings);
 
+/* ---- connected components: the edge-count walk above with one more output, the connected components of every
+ * filter's network, in the same single walk of the pair order and still without returning a pair.
+ *
+ *   - Vertices: the C columns of an all-pairs call; the Cx + Cy columns of [X | Y] for a cross call, X's column i as
+ *     vertex i and Y's column j as vertex Cx + j.
+ *   - Edges of filter f: exactly the pairs n_pass[f] counts.  A diagonal pair (include_diag) is a self-loop and
+ *     changes nothing.
+ *   - Labels: component[c * T + f] (the layout of degree) is the smallest vertex index in c's component under filter
+ *     f.  A column that no edge touches, a degenerate column included, is its own component.  The labels are a
+ *     function of the edge set alone: they do not depend on the window size, the order of the work or the number of
+ *     devices.  A cross call writes x_component[i * T + f] and y_component[j * T + f] (each may be NULL, not both),
+ *     vertex indices into [X | Y].
+ *   - n_components[T] (may be NULL): the number of distinct labels of each filter.
+ *   - Every other argument and output is that of the count call, with the same refusals and messages; a NULL
+ *     component (all-pairs) or both x_component and y_component NULL (cross) is refused too, before any device is
+ *     touched.
+ *   - Device memory adds 4 B x T x V of union-find forest (V vertices) and 8 B x T of counters, whatever the number of
+ *     pairs.  timings: epilogue_ms includes the forest's initialisation (before the first window's tally) and the
+ *     unions; the labels come back once, with the counters, and d2h_ms includes the kernel that resolves them.
+ *   - The _multi twins resolve each device's forest of its slice; the host merges them into the one-device labels. */
+int icikt_all_pairs_components(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                               const icikt_opts* opts, const icikt_edge_filter* filters, int32_t n_filters,
+                               int64_t* n_pass, int64_t* degree, int32_t* component, int64_t* n_components,
+                               int64_t* status_counts, double* max_taumax, icikt_timings* timings);
+int icikt_all_pairs_components_multi(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                                     const icikt_opts* opts, const int32_t* devices, int32_t n_devices,
+                                     const icikt_edge_filter* filters, int32_t n_filters, int64_t* n_pass,
+                                     int64_t* degree, int32_t* component, int64_t* n_components,
+                                     int64_t* status_counts, double* max_taumax, icikt_timings* timings);
+int icikt_cross_components(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                           int32_t n_global_na, const icikt_opts* opts, const icikt_edge_filter* filters,
+                           int32_t n_filters, int64_t* n_pass, int64_t* x_degree, int64_t* y_degree,
+                           int32_t* x_component, int32_t* y_component, int64_t* n_components,
+                           int64_t* status_counts, double* max_taumax, icikt_timings* timings);
+int icikt_cross_components_multi(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
+                                 int32_t n_global_na, const icikt_opts* opts, const int32_t* devices,
+                                 int32_t n_devices, const icikt_edge_filter* filters, int32_t n_filters,
+                                 int64_t* n_pass, int64_t* x_degree, int64_t* y_degree, int32_t* x_component,
+                                 int32_t* y_component, int64_t* n_components, int64_t* status_counts,
+                                 double* max_taumax, icikt_timings* timings);
+
 /* ---- plan API: keeps the matrix, the per-column tables and the results resident in
  * HBM so that repeated runs (benchmarks, several perspectives on one matrix) do not
  * pay the copies.  A plan is bound to one device and is not thread-safe.            */
