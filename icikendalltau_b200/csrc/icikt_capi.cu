@@ -2218,11 +2218,12 @@ static int ensure_cross_buffers(icikt_plan* p) {
   return ICIKT_OK;
 }
 
-// icikt_cross_pairs' walk over pairs [first, last) of the Cx x Cy cross order, into caller arrays indexed from 0 =
+// icikt_cross_pairs' walk over pairs [first, last) of `order` (the cross order), into caller arrays indexed from 0 =
 // first: per window, the results move off the plan's pair buffers into d_cres[b] on the compute stream (the next
 // window's K3 overwrites those buffers), and the host copies them from there into the caller's arrays on the copy
 // stream while the next window computes.
-static int cross_pair_walk(icikt_plan* p, int64_t Cx, int64_t Cy, int64_t first, int64_t last, int64_t W, double* raw,
+template <class Order>
+static int cross_pair_walk(icikt_plan* p, const Order& order, int64_t first, int64_t last, int64_t W, double* raw,
                            double* pvalue, double* taumax, double* completeness, int32_t* status, WalkTotals& tot,
                            float& d2h_ms) {
   const size_t win = (size_t)p->P;
@@ -2253,7 +2254,7 @@ static int cross_pair_walk(icikt_plan* p, int64_t Cx, int64_t Cy, int64_t first,
     d2h_ms += ev_ms(p->ev[6], p->ev[7]);
     return ICIKT_OK;
   };
-  return walk_windows(p, cross_order(Cx, Cy), first, last, W, tot, select, collect);
+  return walk_windows(p, order, first, last, W, tot, select, collect);
 }
 
 // The list rows of a cross top-k call, [c_lo, c_hi) of [X | Y] (X's columns come first, so any choice of sides is one
@@ -2405,6 +2406,22 @@ struct MultiJob {
   bool idle(int k) const { return n_devices > 1 && pair_lo(k + 1) <= pair_lo(k); }  // one of several, without pairs
 };
 
+// An all-pairs job over the whole combn order of s (the diagonal included if o.include_diag), its arguments checked.
+void all_pairs_job(MultiJob& J, const ColumnSource& s, int64_t n, const double* global_na, int32_t n_global_na,
+                   const icikt_opts& o, const int32_t* devices) {
+  J.src = s; J.n = n; J.C = s.C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.ptot = tri_pairs(s.C) + (o.include_diag ? s.C : 0);
+}
+
+// A cross job over pairs [first, last) of the cross order, its arguments checked.  The window plans hold W pairs of
+// a slice: the call's pair range is the job's, not theirs.
+void cross_job(MultiJob& J, const ColumnSource& sx, const ColumnSource& sy, int64_t n, const double* global_na,
+               int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int64_t first, int64_t last) {
+  J.src = sx; J.y = &sy; J.n = n; J.C = sx.C + sy.C; J.global_na = global_na; J.n_global_na = n_global_na;
+  J.devices = devices; J.base = o; J.base.pair_lo = J.base.pair_hi = 0;
+  J.first = first; J.ptot = last - first;
+}
+
 void multi_probe_peers(MultiJob& J) {
   bool distinct = true;
   J.peers_ok = true;
@@ -2433,9 +2450,26 @@ int enable_peers(const MultiJob& J, int k) {
   return ICIKT_OK;
 }
 
+// The peer phase of worker k, once its part is on its device (rc: how that went): it publishes its plan p, or null
+// if it failed, and waits until every worker has.  If every worker succeeded it enables peer access and runs body(),
+// which reads the other workers' buffers in place (J.peer_plan); otherwise it fails with `peer_failed`.  Then it waits
+// until every worker is done, so that nobody's buffers are touched (or freed) while a peer still reads them.  Every
+// worker passes both barriers whatever happened to it, so nobody is left waiting.
+template <class Body>
+int peer_phase(MultiJob& J, int k, icikt_plan* p, int rc, const char* peer_failed, Body&& body) {
+  J.peer_plan[(size_t)k] = (rc == ICIKT_OK) ? p : nullptr;
+  J.barrier.wait();
+  bool all_ok = true;
+  for (int j = 0; j < J.n_devices; ++j) all_ok = all_ok && J.peer_plan[(size_t)j] != nullptr;
+  if (rc == ICIKT_OK && !all_ok) rc = fail(ICIKT_ERR_CUDA, peer_failed);
+  if (rc == ICIKT_OK) rc = enable_peers(J, k);
+  if (rc == ICIKT_OK) rc = body();
+  J.barrier.wait();
+  return rc;
+}
+
 // The column phase of worker k on its plan p (rc: how getting the plan went): sharded K1 and the peer gather of the
-// tables in gather mode, otherwise the upload and K1 of all columns (skipped by an idle worker).  In
-// gather mode every worker passes both barriers whatever happened to it, so nobody is left waiting.  A cross job's
+// tables in gather mode, otherwise the upload and K1 of all columns (skipped by an idle worker).  A cross job's
 // columns are those of [X | Y]: a shard that straddles column Cx uploads X's part, then Y's (upload_span).
 int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
   if (!J.gather) return J.idle(k) || rc != ICIKT_OK ? rc : window_columns(p, J.src, J.global_na, J.n_global_na, J.y);
@@ -2444,33 +2478,27 @@ int multi_worker_columns(MultiJob& J, int k, icikt_plan* p, int rc) {
   if (rc == ICIKT_OK) rc = icikt_plan_columns_range(p, J.global_na, J.n_global_na, J.col_lo(k), J.col_lo(k + 1));
   if (rc == ICIKT_OK) p->tm.n_launches += x_launches;
   if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "column slice");
-  J.peer_plan[(size_t)k] = (rc == ICIKT_OK) ? p : nullptr;
-  J.barrier.wait();  // every slice of the tables is complete on its device
-  bool all_ok = true;
-  for (int j = 0; j < J.n_devices; ++j) all_ok = all_ok && J.peer_plan[(size_t)j] != nullptr;
-  if (rc == ICIKT_OK && !all_ok) rc = fail(ICIKT_ERR_CUDA, "a peer device failed to preprocess its slice");
-  if (rc == ICIKT_OK) rc = enable_peers(J, k);
-  if (rc == ICIKT_OK) {
+  return peer_phase(J, k, p, rc, "a peer device failed to preprocess its slice", [&]() -> int {
     const int dev = J.device_of(k);
     icikt_table mine[ICIKT_MAX_TABLES], theirs[ICIKT_MAX_TABLES];
     const int nt = icikt_plan_tables(p, mine, ICIKT_MAX_TABLES);
-    for (int j = 0; j < J.n_devices && rc == ICIKT_OK; ++j) {
+    int r = ICIKT_OK;
+    for (int j = 0; j < J.n_devices && r == ICIKT_OK; ++j) {
       if (j == k) continue;
       icikt_plan_tables(J.peer_plan[(size_t)j], theirs, ICIKT_MAX_TABLES);
-      for (int t = 0; t < nt && rc == ICIKT_OK; ++t) {
+      for (int t = 0; t < nt && r == ICIKT_OK; ++t) {
         const size_t off = (size_t)J.col_lo(j) * (size_t)mine[t].bytes_per_column;
         const size_t len = (size_t)(J.col_lo(j + 1) - J.col_lo(j)) * (size_t)mine[t].bytes_per_column;
         if (len && cudaMemcpyPeerAsync(static_cast<unsigned char*>(mine[t].ptr) + off, dev,
                                        static_cast<const unsigned char*>(theirs[t].ptr) + off, J.device_of(j), len,
                                        p->stream) != cudaSuccess)
-          rc = cuda_fail(cudaGetLastError(), "cudaMemcpyPeerAsync");
+          r = cuda_fail(cudaGetLastError(), "cudaMemcpyPeerAsync");
       }
     }
-    if (rc == ICIKT_OK) rc = icikt_plan_columns_finish(p);
-    if (rc == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = cuda_fail(cudaGetLastError(), "peer gather");
-  }
-  J.barrier.wait();  // nobody's tables are touched (or freed) before every pull has finished
-  return rc;
+    if (r == ICIKT_OK) r = icikt_plan_columns_finish(p);
+    if (r == ICIKT_OK && cudaStreamSynchronize(p->stream) != cudaSuccess) r = cuda_fail(cudaGetLastError(), "peer gather");
+    return r;
+  });
 }
 
 // The cached plans of a per-pair job's workers, as window_slots: one worker takes g_cached, several one slot each.
@@ -2486,8 +2514,8 @@ int pairs_job(MultiJob& J, const ColumnSource& s, int64_t n, int64_t C, const do
   const int64_t all = tri_pairs(C) + (o.include_diag ? C : 0);
   const int64_t lo = o.pair_lo, hi = (o.pair_lo == 0 && o.pair_hi == 0) ? all : o.pair_hi;
   if (!pi && (lo < 0 || hi > all || lo > hi)) return fail(ICIKT_ERR_BAD_ARG, "pair_lo/pair_hi out of range");
-  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.pi = pi; J.pj = pj; J.devices = devices; J.base = o;
+  all_pairs_job(J, s, n, global_na, n_global_na, o, devices);
+  J.pi = pi; J.pj = pj;
   J.first = pi ? 0 : lo;
   J.ptot = pi ? P : hi - lo;
   return ICIKT_OK;
@@ -2642,7 +2670,6 @@ int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* glo
   std::vector<MultiWork> work;
   std::vector<int32_t> good((size_t)C, 0);
   if (n_good) std::copy(n_good, n_good + C, good.begin());
-  std::vector<icikt_plan*> plans((size_t)n_dev, nullptr);
   rc = run_workers(J, slots, work, max_taumax, timings, [&](int k, MultiWork& w) -> int {
     icikt_plan* p = nullptr;
     w.rc = pairs_worker(J, k, slots, staged, nullptr, &p, nullptr);
@@ -2664,17 +2691,10 @@ int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* glo
       w.rc = icikt_plan_column_info(p, good.data());
       for (int64_t c = 0; c < C && w.rc == ICIKT_OK; ++c) good[(size_t)c] = (int32_t)n - good[(size_t)c];
     }
-    plans[(size_t)k] = (w.rc == ICIKT_OK) ? p : nullptr;
-    J.barrier.wait();  // every slice of the pair results is complete on its device
-    bool all_ok = true;
-    double mx = std::nan("");
-    for (int j = 0; j < n_dev; ++j) {
-      all_ok = all_ok && plans[(size_t)j] != nullptr;
-      if (work[(size_t)j].mx == work[(size_t)j].mx && !(mx >= work[(size_t)j].mx)) mx = work[(size_t)j].mx;
-    }
-    if (w.rc == ICIKT_OK && !all_ok) w.rc = fail(ICIKT_ERR_CUDA, "a peer device failed to compute its pairs");
-    if (w.rc == ICIKT_OK) w.rc = enable_peers(J, k);
-    if (w.rc == ICIKT_OK) w.rc = [&]() -> int {
+    return peer_phase(J, k, p, w.rc, "a peer device failed to compute its pairs", [&]() -> int {
+      double mx = std::nan("");
+      for (const MultiWork& v : work)
+        if (v.mx == v.mx && !(mx >= v.mx)) mx = v.mx;
       const int64_t c_lo = J.col_lo(k), c_hi = J.col_lo(k + 1);
       const size_t blk = (size_t)C * (size_t)(c_hi - c_lo);
       CK(cudaSetDevice(p->device));
@@ -2686,7 +2706,7 @@ int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* glo
       BlockFill f{};
       f.n_dev = n_dev;
       for (int j = 0; j < n_dev; ++j) {
-        const icikt_plan* q = plans[(size_t)j];
+        const icikt_plan* q = J.peer_plan[(size_t)j];
         f.tau[j] = q->d_tau; f.pvalue[j] = q->d_p; f.taumax[j] = q->d_tm; f.completeness[j] = q->d_comp;
         f.status[j] = q->d_status;
         f.pair_lo[j] = J.pair_lo(j);
@@ -2715,9 +2735,7 @@ int matrices_impl(const ColumnSource& s, int64_t n, int64_t C, const double* glo
       CK(cudaEventRecord(p->ev[7], p->stream));
       CK(cudaStreamSynchronize(p->stream));
       return icikt_plan_timings(p, &w.tm);
-    }();
-    J.barrier.wait();  // nobody's results are freed before every block has been filled
-    return w.rc;
+    });
   });
   icikt_plan_destroy(list_plan);
   if (rc != ICIKT_OK || n_dev == 1) return rc;
@@ -2748,6 +2766,15 @@ int check_window_devices(int32_t n_devices) {
   return ICIKT_OK;
 }
 
+// The matrix x of an all-pairs call that takes an icikt_input, and the arguments the windowed calls share, checked
+// before any device is touched.
+int check_all_pairs_input(const icikt_input* x, int64_t n, const double* global_na, int32_t n_global_na,
+                          const icikt_opts& o, int32_t n_devices, ColumnSource* s) {
+  int rc = n < 1 ? fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1") : cross_source(x, "x", n, s);
+  if (rc == ICIKT_OK) rc = check_window_args(*s, n, s->C, global_na, n_global_na, o);
+  return rc == ICIKT_OK ? check_window_devices(n_devices) : rc;
+}
+
 // The cached window plans of J's workers: one worker takes the single-device slot, several take one slot each, so
 // that one-device and multi-device calls alternated on the same data do not reallocate each other's plans.
 icikt_plan** window_slots(const MultiJob& J) { return J.n_devices == 1 ? &g_cached_edges : g_cached_wmulti; }
@@ -2764,17 +2791,45 @@ int window_multi_worker(MultiJob& J, int k, icikt_plan** out) {
   return rc;
 }
 
-// walk(order) with the pair order of J's walk: the cross order of a cross job, the combn order of p otherwise
+// The windowed job J, its arguments checked.  Worker k takes its window plan p and runs the column phase
+// (window_multi_worker); walk(k, p, order, lo, hi, tot, d2h_ms) then reserves its buffers and walks its slice [lo, hi)
+// of J's pair order (`order`: the cross order of a cross job, the combn order otherwise), d2h_ms receiving the time
+// of its copies out, and finish_walk gives its timings.  An idle worker walks nothing.  *M receives the maximum
+// taumax over all pairs; a job without pairs walks nothing and leaves *M NaN and the timings zero.
+// `merge` (the top-k lists, merged on the devices): devices that cannot read each other's lists make the job one
+// worker on devices[0]; of several workers, every one then runs merge(k, p, rc, tm) whatever its rc, and an idle
+// worker walks its empty slice too, so that the merge reads empty lists.
 template <class Walk>
-int with_order(const MultiJob& J, const icikt_plan* p, Walk&& walk) {
-  return J.y ? walk(cross_order(J.src.C, J.y->C)) : walk(combn_order(p));
-}
-
-// the result of a job without pairs: no maximum, no time
-int no_pairs(double* max_taumax, icikt_timings* timings) {
-  if (max_taumax) *max_taumax = std::nan("");
-  if (timings) std::memset(timings, 0, sizeof(*timings));
-  return ICIKT_OK;
+int run_windows(MultiJob& J, double* M, icikt_timings* timings, Walk&& walk,
+                const std::function<int(int, icikt_plan*, int, icikt_timings&)>& merge = nullptr) {
+  int rc = select_device(J.device_of(0));
+  if (rc != ICIKT_OK) return rc;
+  *M = std::nan("");
+  if (J.ptot == 0) {  // one column without the diagonal, or an empty cross range: nothing to compute
+    if (timings) std::memset(timings, 0, sizeof(*timings));
+    return ICIKT_OK;
+  }
+  std::vector<MultiWork> work;
+  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
+  std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
+  multi_probe_peers(J);
+  if (merge && !J.peers_ok) J.n_devices = 1;
+  rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
+    icikt_plan* p = nullptr;
+    int r = window_multi_worker(J, k, &p);
+    if (r == ICIKT_OK && (merge || !J.idle(k))) {
+      WalkTotals tot;
+      float d2h_ms = 0.f;
+      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
+      auto walk_on = [&](const auto& order) { return walk(k, p, order, lo, hi, tot, d2h_ms); };
+      r = J.y ? walk_on(cross_order(J.src.C, J.y->C)) : walk_on(combn_order(p));
+      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
+      bits[(size_t)k] = tot.bits;
+    }
+    return merge && J.n_devices > 1 ? merge(k, p, r, w.tm) : r;
+  });
+  if (rc == ICIKT_OK) *M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  return rc;
 }
 
 // The adjusted p-values of the rows held (the _padj calls), once every worker has walked its slice: m is the sum of
@@ -2905,16 +2960,6 @@ int padj_finish(const MultiJob& J, std::vector<PadjPart>& parts, const icikt_pad
 // (the _padj calls), every worker also keeps its candidates, and padj_finish gives the rows their adjusted values.
 int edges_run(MultiJob& J, const icikt_edge_filter& f0, icikt_edges** out, double* max_taumax, icikt_timings* timings,
               const icikt_padj_filter* adjust = nullptr) {
-  int rc = select_device(J.device_of(0));
-  if (rc != ICIKT_OK) return rc;
-  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
-  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
-  res->j_offset = J.y ? (int32_t)J.src.C : 0;
-  if (adjust) res->n_tests = 0;
-  if (J.ptot == 0) {  // one column, no diagonal: nothing to compute
-    *out = res.release();
-    return no_pairs(max_taumax, timings);
-  }
   // The candidate bound: every row with padj <= max_padj has p <= max_padj (icikt_padj.cuh).  A max_padj >= 1 keeps
   // every row, as does NaN.  The rows take it as one more p-value bound.
   icikt_edge_filter f = f0;
@@ -2924,32 +2969,19 @@ int edges_run(MultiJob& J, const icikt_edge_filter& f0, icikt_edges** out, doubl
     for (PadjPart& pt : parts) pt.bound = b;
     if (b == b && !(f.max_pvalue <= b)) f.max_pvalue = b;
   }
-  std::vector<MultiWork> work;
   std::vector<std::vector<EdgeRow>> rows((size_t)J.n_devices);
-  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
   EdgeHeld held;
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
-    multi_probe_peers(J);
-    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
-      icikt_plan* p = nullptr;
-      int r = window_multi_worker(J, k, &p);
-      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
-      if (r != ICIKT_OK || hi <= lo) return r;
-      WalkTotals tot;
-      float d2h_ms = 0.f;
-      r = ensure_edge_buffers(p, p->P);
-      if (r == ICIKT_OK)
-        r = with_order(J, p, [&](const auto& order) {
-          return edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms,
-                           adjust ? &parts[(size_t)k] : nullptr);
-        });
-      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
-      bits[(size_t)k] = tot.bits;
-      return r;
-    });
-  }
+  double M;
+  int rc = run_windows(J, &M, timings, [&](int k, icikt_plan* p, const auto& order, int64_t lo, int64_t hi,
+                                           WalkTotals& tot, float& d2h_ms) {
+    const int r = ensure_edge_buffers(p, p->P);
+    return r != ICIKT_OK ? r : edge_walk(p, order, f, lo, hi, p->P, rows[(size_t)k], held, tot, d2h_ms,
+                                         adjust ? &parts[(size_t)k] : nullptr);
+  });
   if (rc != ICIKT_OK) return rc;
+  std::unique_ptr<icikt_edges> res(new (std::nothrow) icikt_edges());
+  if (!res) return fail(ICIKT_ERR_ALLOC, "out of host memory");
+  res->j_offset = J.y ? (int32_t)J.src.C : 0;
   size_t total = 0;
   for (const auto& r : rows) total += r.size();
   res->rows = std::move(rows[0]);
@@ -2962,7 +2994,6 @@ int edges_run(MultiJob& J, const icikt_edge_filter& f0, icikt_edges** out, doubl
     res->rows.insert(res->rows.end(), rows[k].begin(), rows[k].end());
     std::vector<EdgeRow>().swap(rows[k]);
   }
-  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
   float padj_ms = 0.f;
   rc = edge_result(res.get(), f, M, adjust ? [&](icikt_edges* e) { return padj_finish(J, parts, *adjust, e, &padj_ms); }
                                            : std::function<int(icikt_edges*)>());
@@ -2983,8 +3014,7 @@ int edges_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global
   if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
-  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.ptot = tri_pairs(C) + (o.include_diag ? C : 0);
+  all_pairs_job(J, s, n, global_na, n_global_na, o, devices);
   return edges_run(J, *filter, out, max_taumax, timings);
 }
 
@@ -3017,11 +3047,11 @@ int topk_copy_lists(icikt_plan* p, int64_t L, int K, const std::vector<TopkSide>
 }
 
 // Worker k's block of list rows [L*k/N, L*(k+1)/N) of the merged lists (L rows: the columns of an all-pairs call,
-// the requested sides of a cross call): the merge kernel reads every device's lists in place, and the block goes
-// straight into the caller's arrays of every side it covers (one block may hold rows of both sides of a cross
-// call); held[r] receives row r's entries.  tm: the merge and its copies become d2h_ms.
-int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<icikt_plan*>& plans, int64_t L, int K,
-                     int by, const std::vector<TopkSide>& sides, int32_t* held, icikt_timings& tm) {
+// the requested sides of a cross call): the merge kernel reads every device's lists in place (J.peer_plan), and the
+// block goes straight into the caller's arrays of every side it covers (one block may hold rows of both sides of a
+// cross call); held[r] receives row r's entries.  tm: the merge and its copies become d2h_ms.
+int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, int64_t L, int K, int by,
+                     const std::vector<TopkSide>& sides, int32_t* held, icikt_timings& tm) {
   const int64_t r_lo = L * k / J.n_devices, r_hi = L * (k + 1) / J.n_devices;
   if (r_hi <= r_lo) return ICIKT_OK;
   const size_t blk = (size_t)(r_hi - r_lo) * (size_t)K;
@@ -3030,9 +3060,9 @@ int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<
   TopkDeviceMerge m{};
   m.n_dev = J.n_devices;
   for (int j = 0; j < J.n_devices; ++j) {
-    m.col[j] = plans[(size_t)j]->d_tcol.get();
-    m.idx[j] = plans[(size_t)j]->d_tidx.get();
-    m.list[j] = plans[(size_t)j]->d_tlist.get();
+    m.col[j] = J.peer_plan[(size_t)j]->d_tcol.get();
+    m.idx[j] = J.peer_plan[(size_t)j]->d_tidx.get();
+    m.list[j] = J.peer_plan[(size_t)j]->d_tlist.get();
   }
   m.C = L;  // the lists' rows: the kernel's columns
   m.c_lo = r_lo;
@@ -3068,63 +3098,37 @@ int topk_merge_block(const MultiJob& J, int k, icikt_plan* p, const std::vector<
 }
 
 // The top-k call over the devices of J, its arguments checked: every worker keeps the lists of rows [c_lo, c_hi)
-// (columns of the plan) for its slice.  One worker copies its lists out (topk_copy_lists); several merge a block of
-// rows each into the sides' arrays after a barrier (topk_merge_block).  Then the host shifts the partners and pads
-// (topk_sides_finish).
+// (columns of the plan) for its slice.  One worker copies its lists out (topk_copy_lists) before its walk is
+// finished; several merge a block of rows each into the sides' arrays in a peer phase after it (topk_merge_block).
+// Then the host shifts the partners and pads (topk_sides_finish).
 int topk_run(MultiJob& J, int K, int by, bool scale, int64_t c_lo, int64_t c_hi, std::vector<TopkSide>& sides,
              double* max_taumax, icikt_timings* timings) {
-  int rc = select_device(J.device_of(0));
+  int rc = ICIKT_OK;
   for (TopkSide& sd : sides)
     if (rc == ICIKT_OK) rc = topk_raw_buffer(sd.out, sd.cols * K, sd.raw_own, &sd.raw);
   if (rc != ICIKT_OK) return rc;
-  if (J.ptot == 0) {  // one column: no candidate, its list is padding
-    topk_sides_finish(sides, K, [](int64_t) { return 0; }, scale, std::nan(""));
-    return no_pairs(max_taumax, timings);
-  }
   const int64_t L = c_hi - c_lo;
-  std::vector<int32_t> held;
+  std::vector<int32_t> held;  // without pairs (one column) every list stays empty: padding
   try {
     held.resize((size_t)L);
   } catch (const std::bad_alloc&) {
     return fail(ICIKT_ERR_ALLOC, "out of host memory for the lists");
   }
-  std::vector<MultiWork> work;
-  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
-  std::vector<icikt_plan*> plans((size_t)J.n_devices, nullptr);
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
-    multi_probe_peers(J);
-    // devices that cannot read each other's lists: one worker on devices[0] (no gather, no barrier)
-    if (!J.peers_ok) J.n_devices = 1;
-    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
-      icikt_plan* p = nullptr;
-      int r = window_multi_worker(J, k, &p);
-      WalkTotals tot;
-      if (r == ICIKT_OK) r = ensure_topk_buffers(p, p->P, K, L);
-      if (r == ICIKT_OK)
-        r = with_order(J, p, [&](const auto& order) {
-          return topk_walk(p, order, c_lo, c_hi, K, by, J.pair_lo(k), J.pair_lo(k + 1), p->P, tot);
+  double M;
+  rc = run_windows(
+      J, &M, timings,
+      [&](int, icikt_plan* p, const auto& order, int64_t lo, int64_t hi, WalkTotals& tot, float& d2h_ms) {
+        int r = ensure_topk_buffers(p, p->P, K, L);
+        if (r == ICIKT_OK) r = topk_walk(p, order, c_lo, c_hi, K, by, lo, hi, p->P, tot);
+        if (r == ICIKT_OK && J.n_devices == 1) r = topk_copy_lists(p, L, K, sides, held.data(), &d2h_ms);
+        return r;
+      },
+      [&](int k, icikt_plan* p, int r, icikt_timings& tm) {
+        return peer_phase(J, k, p, r, "a peer device failed to select its lists", [&] {
+          return topk_merge_block(J, k, p, L, K, by, sides, held.data(), tm);
         });
-      bits[(size_t)k] = tot.bits;
-      if (J.n_devices == 1) {
-        float d2h_ms = 0.f;
-        if (r == ICIKT_OK) r = topk_copy_lists(p, L, K, sides, held.data(), &d2h_ms);
-        return r == ICIKT_OK ? finish_walk(p, tot, d2h_ms, &w.tm) : r;
-      }
-      if (r == ICIKT_OK) r = finish_walk(p, tot, 0.f, &w.tm);
-      plans[(size_t)k] = (r == ICIKT_OK) ? p : nullptr;
-      J.barrier.wait();  // every device's lists are complete
-      bool all_ok = true;
-      for (int j = 0; j < J.n_devices; ++j) all_ok = all_ok && plans[(size_t)j] != nullptr;
-      if (r == ICIKT_OK && !all_ok) r = fail(ICIKT_ERR_CUDA, "a peer device failed to select its lists");
-      if (r == ICIKT_OK) r = enable_peers(J, k);
-      if (r == ICIKT_OK) r = topk_merge_block(J, k, p, plans, L, K, by, sides, held.data(), w.tm);
-      J.barrier.wait();  // nobody's lists are freed (or reused) before every block has been merged
-      return r;
-    });
-  }
+      });
   if (rc != ICIKT_OK) return rc;
-  const double M = max_of_bits(*std::max_element(bits.begin(), bits.end()));
   topk_sides_finish(sides, K, [&](int64_t row) { return held[(size_t)row]; }, scale, M);
   if (max_taumax) *max_taumax = M;
   return ICIKT_OK;
@@ -3137,22 +3141,12 @@ int topk_impl(const ColumnSource& s, int64_t n, int64_t C, const double* global_
   if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
-  J.src = s; J.n = n; J.C = C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.ptot = tri_pairs(C);
+  all_pairs_job(J, s, n, global_na, n_global_na, o, devices);
   std::vector<TopkSide> sides{TopkSide{out, 0, C, 0, {}, nullptr}};
   return topk_run(J, K, by, scale_max != 0, 0, C, sides, max_taumax, timings);
 }
 
 // ---- the cross calls: the cross order (of the call's range) sliced as above over the Cx + Cy columns of [X | Y]
-
-// A cross job over pairs [first, last) of the cross order, its arguments checked.  The window plans hold W pairs of
-// a slice: the call's pair range is the job's, not theirs.
-void cross_job(MultiJob& J, const ColumnSource& sx, const ColumnSource& sy, int64_t n, const double* global_na,
-               int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int64_t first, int64_t last) {
-  J.src = sx; J.y = &sy; J.n = n; J.C = sx.C + sy.C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.base.pair_lo = J.base.pair_hi = 0;
-  J.first = first; J.ptot = last - first;
-}
 
 int cross_pairs_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
                      int32_t n_global_na, const icikt_opts& o, const int32_t* devices, int32_t n_devices, double* raw,
@@ -3166,34 +3160,19 @@ int cross_pairs_impl(const icikt_input* x, const icikt_input* y, int64_t n, cons
   const int64_t first = o.pair_lo, last = (o.pair_hi == 0) ? sx.C * sy.C : o.pair_hi;
   MultiJob J(n_devices);
   cross_job(J, sx, sy, n, global_na, n_global_na, o, devices, first, last);
-  rc = select_device(J.device_of(0));
-  if (rc != ICIKT_OK) return rc;
-  if (J.ptot == 0) return no_pairs(max_taumax, timings);  // an empty slice
-  std::vector<MultiWork> work;
-  std::vector<unsigned long long> bits((size_t)n_devices, 0);
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
-    multi_probe_peers(J);
-    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
-      icikt_plan* p = nullptr;
-      int r = window_multi_worker(J, k, &p);
-      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1), off = lo - first;
-      if (r != ICIKT_OK || hi <= lo) return r;
-      WalkTotals tot;
-      float d2h_ms = 0.f;
-      r = ensure_cross_buffers(p);
-      if (r == ICIKT_OK)
-        r = cross_pair_walk(p, sx.C, sy.C, lo, hi, p->P, raw + off, pvalue ? pvalue + off : nullptr,
-                            taumax ? taumax + off : nullptr, completeness ? completeness + off : nullptr,
-                            status ? status + off : nullptr, tot, d2h_ms);
-      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
-      bits[(size_t)k] = tot.bits;
-      return r;
-    });
-  }
-  if (rc != ICIKT_OK) return rc;
-  if (max_taumax) *max_taumax = max_of_bits(*std::max_element(bits.begin(), bits.end()));
-  return ICIKT_OK;
+  double M;
+  rc = run_windows(J, &M, timings, [&](int, icikt_plan* p, const auto& order, int64_t lo, int64_t hi,
+                                       WalkTotals& tot, float& d2h_ms) {
+    const int64_t off = lo - first;
+    const int r = ensure_cross_buffers(p);
+    return r != ICIKT_OK ? r
+                         : cross_pair_walk(p, order, lo, hi, p->P, raw + off, pvalue ? pvalue + off : nullptr,
+                                           taumax ? taumax + off : nullptr,
+                                           completeness ? completeness + off : nullptr,
+                                           status ? status + off : nullptr, tot, d2h_ms);
+  });
+  if (rc == ICIKT_OK && max_taumax) *max_taumax = M;
+  return rc;
 }
 
 int cross_edges_impl(const icikt_input* x, const icikt_input* y, int64_t n, const double* global_na,
@@ -3252,13 +3231,10 @@ int edges_padj_impl(const icikt_input* x, int64_t n, const double* global_na, in
   ColumnSource s;
   int rc = check_filter_args(filter, out);
   if (rc == ICIKT_OK) rc = check_padj(adjust);
-  if (rc == ICIKT_OK) rc = n < 1 ? fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1") : cross_source(x, "x", n, &s);
-  if (rc == ICIKT_OK) rc = check_window_args(s, n, s.C, global_na, n_global_na, o);
-  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc == ICIKT_OK) rc = check_all_pairs_input(x, n, global_na, n_global_na, o, n_devices, &s);
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
-  J.src = s; J.n = n; J.C = s.C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.ptot = tri_pairs(s.C) + (o.include_diag ? s.C : 0);
+  all_pairs_job(J, s, n, global_na, n_global_na, o, devices);
   return edges_run(J, *filter, out, max_taumax, timings, adjust);
 }
 
@@ -3308,35 +3284,15 @@ int check_count_filters(const icikt_edge_filter* filters, int32_t n_filters, con
 int count_run(MultiJob& J, const CountSpec& cs, int64_t* n_pass, const std::vector<DegreeOut>& deg,
               int64_t* status_counts, double* max_taumax, icikt_timings* timings,
               const std::vector<ComponentOut>& comp = {}, int64_t* n_components = nullptr) {
-  int rc = select_device(J.device_of(0));
-  if (rc != ICIKT_OK) return rc;
-  std::vector<std::vector<unsigned long long>> got((size_t)J.n_devices);
+  std::vector<std::vector<unsigned long long>> got((size_t)J.n_devices);  // without pairs every count is 0
   std::vector<std::vector<int32_t>> labels((size_t)J.n_devices);
-  std::vector<unsigned long long> bits((size_t)J.n_devices, 0);
-  if (J.ptot > 0) {
-    std::vector<MultiWork> work;
-    std::lock_guard<std::mutex> lock(g_cache_mu);  // the cached plans are not re-entrant
-    multi_probe_peers(J);
-    rc = run_workers(J, window_slots(J), work, nullptr, timings, [&](int k, MultiWork& w) -> int {
-      icikt_plan* p = nullptr;
-      int r = window_multi_worker(J, k, &p);
-      const int64_t lo = J.pair_lo(k), hi = J.pair_lo(k + 1);
-      if (r != ICIKT_OK || hi <= lo) return r;
-      WalkTotals tot;
-      float d2h_ms = 0.f;
-      r = ensure_walk_buffers(p);
-      if (r == ICIKT_OK)
-        r = with_order(J, p, [&](const auto& order) {
-          return count_walk(p, order, cs, lo, hi, p->P, tot, got[(size_t)k], labels[(size_t)k], d2h_ms);
-        });
-      if (r == ICIKT_OK) r = finish_walk(p, tot, d2h_ms, &w.tm);
-      bits[(size_t)k] = tot.bits;
-      return r;
-    });
-    if (rc != ICIKT_OK) return rc;
-  } else {
-    no_pairs(max_taumax, timings);  // one column, no diagonal: every count is 0
-  }
+  double M;
+  const int rc = run_windows(J, &M, timings, [&](int k, icikt_plan* p, const auto& order, int64_t lo, int64_t hi,
+                                                 WalkTotals& tot, float& d2h_ms) {
+    const int r = ensure_walk_buffers(p);
+    return r != ICIKT_OK ? r : count_walk(p, order, cs, lo, hi, p->P, tot, got[(size_t)k], labels[(size_t)k], d2h_ms);
+  });
+  if (rc != ICIKT_OK) return rc;
   const int T = cs.T;
   const int64_t C = J.C;
   auto sum = [&](size_t at) {
@@ -3352,7 +3308,7 @@ int count_run(MultiJob& J, const CountSpec& cs, int64_t* n_pass, const std::vect
     if (d.out)
       for (int64_t c = d.c_lo; c < d.c_hi; ++c)
         for (int f = 0; f < T; ++f) d.out[(c - d.c_lo) * T + f] = sum(16 + (size_t)T + (size_t)f * (size_t)C + (size_t)c);
-  if (J.ptot > 0 && max_taumax) *max_taumax = max_of_bits(*std::max_element(bits.begin(), bits.end()));
+  if (max_taumax) *max_taumax = M;
   if (!cs.components) return ICIKT_OK;
   std::vector<const int32_t*> walked;  // the devices that walked pairs
   const std::vector<unsigned long long>* hooks = nullptr;
@@ -3395,13 +3351,10 @@ int count_edges_impl(const icikt_input* x, int64_t n, const double* global_na, i
   int rc = check_count_filters(filters, n_filters, n_pass, degree != nullptr, &cs);
   cs.components = components;
   if (rc == ICIKT_OK && components && !component) rc = fail(ICIKT_ERR_BAD_ARG, "component is NULL");
-  if (rc == ICIKT_OK) rc = n < 1 ? fail(ICIKT_ERR_BAD_ARG, "n and C must be >= 1") : cross_source(x, "x", n, &s);
-  if (rc == ICIKT_OK) rc = check_window_args(s, n, s.C, global_na, n_global_na, o);
-  if (rc == ICIKT_OK) rc = check_window_devices(n_devices);
+  if (rc == ICIKT_OK) rc = check_all_pairs_input(x, n, global_na, n_global_na, o, n_devices, &s);
   if (rc != ICIKT_OK) return rc;
   MultiJob J(n_devices);
-  J.src = s; J.n = n; J.C = s.C; J.global_na = global_na; J.n_global_na = n_global_na;
-  J.devices = devices; J.base = o; J.ptot = tri_pairs(s.C) + (o.include_diag ? s.C : 0);
+  all_pairs_job(J, s, n, global_na, n_global_na, o, devices);
   return count_run(J, cs, n_pass, {DegreeOut{degree, 0, s.C}}, status_counts, max_taumax, timings,
                    {ComponentOut{component, 0, s.C}}, n_components);
 }
